@@ -24,7 +24,7 @@ FRONT_PATH = os.path.join(CSRC, "libcrtfront.so")
 
 INVALID = 0xFFFFFFFF
 MAT_DIFFUSE, MAT_REFLECTIVE, MAT_CONSTANT, MAT_REFRACTIVE = 0, 1, 2, 3
-RAY_PRIMARY, RAY_SHADOW, RAY_REFLECTION, RAY_REFRACTION = 0, 1, 2, 3
+RAY_PRIMARY, RAY_SHADOW, RAY_REFLECTION, RAY_REFRACTION, RAY_DIFFUSE = 0, 1, 2, 3, 4
 # RenderOptimization (RayTracer.h:12-23) + the new enumerator
 MODE_BVH_BUCKETS_THREADPOOL = 8
 MODE_B200_WAVEFRONT = 10
@@ -123,6 +123,21 @@ class Stats(C.Structure):
         return d
 
 
+class Sampling(C.Structure):
+    """crtb200_sampling: GI + jittered supersampling under the project's sampling contract (DESIGN.md 3.10)."""
+    _fields_ = [("use_gi", C.c_uint32), ("gi_samples", C.c_uint32), ("rays_per_pixel", C.c_uint32),
+                ("monte_carlo_bias", C.c_float), ("seed", C.c_uint32), ("frame_index", C.c_uint32)]
+
+    @staticmethod
+    def make(use_gi: bool = True, gi_samples: int = 2, rays_per_pixel: int = 1, monte_carlo_bias: float = 1e-4,
+             seed: int = 0, frame_index: int = 0) -> "Sampling":
+        return Sampling(1 if use_gi else 0, gi_samples, rays_per_pixel, monte_carlo_bias, seed, frame_index)
+
+
+class SamplingStats(C.Structure):
+    _fields_ = [("rays_diffuse", C.c_uint64), ("samples", C.c_uint32), ("reserved", C.c_uint32)]
+
+
 class SceneInfo(C.Structure):
     _fields_ = [("width", C.c_uint32), ("height", C.c_uint32), ("bucket_size", C.c_uint32), ("n_meshes", C.c_uint32),
                 ("n_materials", C.c_uint32), ("n_textures", C.c_uint32), ("n_lights", C.c_uint32),
@@ -173,6 +188,8 @@ def core() -> C.CDLL:
         lib.crtb200_trace_rays.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]
         lib.crtb200_device_count.argtypes = [C.POINTER(C.c_int)]
         lib.crtb200_debug_powf5.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]
+        lib.crtb200_set_sampling.argtypes = [C.c_void_p, C.POINTER(Sampling)]
+        lib.crtb200_last_sampling_stats.argtypes = [C.c_void_p, C.POINTER(SamplingStats)]
         _core = lib
     return _core
 
@@ -203,6 +220,8 @@ def front() -> C.CDLL:
         lib.crtfe_tracer_set_camera.argtypes = [C.c_void_p, C.POINTER(Camera)]
         lib.crtfe_tracer_get_camera.argtypes = [C.c_void_p, C.POINTER(Camera)]
         lib.crtfe_tracer_render.argtypes = [C.c_void_p, C.c_char_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.POINTER(Stats)]
+        lib.crtfe_tracer_render_sampled.argtypes = [C.c_void_p, C.c_char_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32,
+                                                    C.c_uint32, C.c_uint32, C.c_float, C.c_uint32, C.c_void_p, C.POINTER(Stats)]
         _front = lib
     return _front
 
@@ -365,6 +384,19 @@ class Context:
     def set_concurrency(self, chunks_in_flight: int) -> None:
         _check_core(core().crtb200_set_concurrency(self._h, chunks_in_flight))
 
+    def set_sampling(self, sampling: Optional[Sampling] = None, **kw) -> None:
+        """crtb200_set_sampling for every later render of this context: a Sampling, or Sampling.make(**kw) keywords;
+        set_sampling(None) with no keywords turns GI / supersampling off."""
+        if sampling is None and kw:
+            sampling = Sampling.make(**kw)
+        _check_core(core().crtb200_set_sampling(self._h, C.byref(sampling) if sampling is not None else None))
+
+    def sampling_stats(self) -> dict:
+        """{'rays_diffuse', 'samples'} of the last render (crtb200_last_sampling_stats)."""
+        st = SamplingStats()
+        _check_core(core().crtb200_last_sampling_stats(self._h, C.byref(st)))
+        return {"rays_diffuse": st.rays_diffuse, "samples": st.samples}
+
     def render(self, camera: Camera, options: Options, want_rgb: bool = True, want_rgb8: bool = False,
                want_hits: bool = False, rgb_out: Optional[np.ndarray] = None, rgb8_out: Optional[np.ndarray] = None):
         """crtb200_render with host buffers.  Returns (rgb f32 HxWx3 | None, rgb8 | None, hits | None, stats dict)."""
@@ -473,12 +505,20 @@ class RayTracer:
         _check_front(front().crtfe_tracer_get_camera(self._h, C.byref(cam)))
         return cam
 
-    def render(self, path_to_image: str = "", mode: int = MODE_B200_WAVEFRONT, max_depth: int = 5, literal: bool = False):
+    def render(self, path_to_image: str = "", mode: int = MODE_B200_WAVEFRONT, max_depth: int = 5, literal: bool = False,
+               use_gi: bool = False, gi_samples: int = 2, rays_per_pixel: int = 1, seed: int = 0,
+               monte_carlo_bias: float = 1e-4):
+        """use_gi / gi_samples / rays_per_pixel / monte_carlo_bias = RenderOptions' GI members, seed = RenderOptions::SEED."""
         h, w = self.scene.info.height, self.scene.info.width
         rgb = np.zeros((h, w, 3), np.float32)
         st = Stats()
-        _check_front(front().crtfe_tracer_render(self._h, path_to_image.encode(), mode, max_depth, 1 if literal else 0,
-                                                 rgb.ctypes.data, C.byref(st)))
+        if use_gi:
+            _check_front(front().crtfe_tracer_render_sampled(self._h, path_to_image.encode(), mode, max_depth, 1 if literal else 0,
+                                                             1, gi_samples, rays_per_pixel, monte_carlo_bias, seed,
+                                                             rgb.ctypes.data, C.byref(st)))
+        else:
+            _check_front(front().crtfe_tracer_render(self._h, path_to_image.encode(), mode, max_depth, 1 if literal else 0,
+                                                     rgb.ctypes.data, C.byref(st)))
         return rgb, st.as_dict()
 
     def close(self):

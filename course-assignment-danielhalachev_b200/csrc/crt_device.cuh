@@ -213,9 +213,8 @@ CRT_DI void ray_prepare(Ray &r, bool primary) {
 }
 
 // RayTracer::getRay + the second normalisation of shootRay                      RayTracer.cpp:61-80, 420
-CRT_DI void primary_ray(const DCamera &cam, uint32_t W, uint32_t H, uint32_t row, uint32_t col, V3 &o, V3 &d) {
-  float x = fadd((float)col, 0.5f);
-  float y = fadd((float)row, 0.5f);
+// x, y = the pixel position: col + 0.5, row + 0.5, or col + jitter, row + jitter (sampling contract, DESIGN.md 3.10)
+CRT_DI void primary_ray_at(const DCamera &cam, uint32_t W, uint32_t H, float x, float y, V3 &o, V3 &d) {
   x = fdiv(x, (float)W);
   y = fdiv(y, (float)H);
   x = fsub(fmul(2.0f, x), 1.0f);
@@ -228,6 +227,9 @@ CRT_DI void primary_ray(const DCamera &cam, uint32_t W, uint32_t H, uint32_t row
              fadd(fadd(fmul(x, cam.rot[2]), fmul(y, cam.rot[5])), fmul(z, cam.rot[8])));
   d = vnorm(vnorm(dr));
   o = mk(cam.pos[0], cam.pos[1], cam.pos[2]);
+}
+CRT_DI void primary_ray(const DCamera &cam, uint32_t W, uint32_t H, uint32_t row, uint32_t col, V3 &o, V3 &d) {
+  primary_ray_at(cam, W, H, fadd((float)col, 0.5f), fadd((float)row, 0.5f), o, d);
 }
 
 // BoundingBox::hasIntersection                                                  BoundingBox.h:85-108

@@ -18,6 +18,7 @@
 #pragma once
 #include "crt_device.cuh"
 #include "crt_powf5.h"
+#include "crt_sampling.h"
 
 namespace crtd {
 
@@ -43,11 +44,16 @@ struct Frame {
   uint32_t max_depth;
   uint32_t resolve;                   // 1 when the frame has secondary levels: k_resolve will read the combine records
   float shadow_bias, reflection_bias, refraction_bias;
+  // sampling contract (crt_sampling.h, DESIGN.md 3.10).  gi = 0: the unsampled frame, none of the fields below is read
+  uint32_t gi, gi_samples;            // diffuse children per diffuse hit (G)
+  uint32_t sample, spp;               // sample pass of this launch, samples per pixel
+  uint32_t seed, frame_index;         // Philox key
+  float mc_bias;                      // MONTE_CARLO_BIAS: diffuse ray origin = P + N * mc_bias
 };
 
 struct Levels {
-  float4 *ray_o;      // xyz origin, w = parent node (unused)      -- indexed by node id - offset[1]
-  float4 *ray_d;      // xyz direction (normalised twice), w = ray type
+  float4 *ray_o;      // xyz origin, w = parent node (unused; GI frames: bits of the ray's path key)  -- indexed by node id - offset[1]
+  float4 *ray_d;      // xyz direction (normalised twice), w = ray type (GI frames: bits of the global pixel index)
   uint32_t *hit_tri;  // per node: global triangle id or CRT_INVALID
   float *hit_t;
   float4 *color;      // per node: resolved colour
@@ -55,7 +61,7 @@ struct Levels {
   float4 *dq;         // diffuse queue, 3 x float4 per item: {P, bits(node)} {N, base.r} {base.g, base.b, -, -}
   uint8_t *vis;       // per (diffuse item, light): 1 = the light is visible from the hit
   uint32_t *counts;   // [CRT_MAX_LEVELS] rays per level; [CRT_MAX_LEVELS] = diffuse queue length
-  unsigned long long *stats;  // [0..3] rays by type, [4],[5] closest node / triangle tests, [6],[7] shadow, [32],[33] walks handed to k_coop, [40] shadow rays answered without a walk
+  unsigned long long *stats;  // [0..3] rays by type, [4],[5] closest node / triangle tests, [6],[7] shadow, [32],[33] walks handed to k_coop, [40] shadow rays answered without a walk, [41] diffuse rays
   uint32_t offset[CRT_MAX_LEVELS + 1];
   // tail hand-off (k_coop): once the work queue of a traversal kernel is dry, the walks still running are written to
   // ovf[] (3 x uint4 per record) and finished one WARP per ray; tail_iters = 0 switches this off
@@ -71,7 +77,16 @@ struct Levels {
   uint32_t skip_zero_terms;  // 1 (default traversal): shadow rays whose light term is exactly zero are answered without a walk
 };
 
-enum { COMB_FINAL = 0, COMB_REFLECT = 1, COMB_FRESNEL = 2, COMB_COPY = 3 };
+// COMB_GI = {kind, first diffuse child (CRT_INVALID: beyond max_depth, every child is the background), diffuse item, G}
+enum { COMB_FINAL = 0, COMB_REFLECT = 1, COMB_FRESNEL = 2, COMB_COPY = 3, COMB_GI = 4 };
+
+// Jittered primary ray of sample fr.sample of pixel (row, col): r = R(p, s, 0, 0), x = col + unit(r[0]),
+// y = row + unit(r[1]), then getRay unchanged.  Returns the root path key r[2].
+CRT_DI uint32_t jittered_primary_ray(const Frame &fr, uint32_t W, uint32_t H, uint32_t row, uint32_t col, V3 &o, V3 &d) {
+  const crt_s_u4 r = crt_s_philox(row * W + col, fr.sample, 0u, 0u, fr.seed, fr.frame_index);
+  primary_ray_at(fr.cam, W, H, fadd((float)col, crt_s_unit(r.x)), fadd((float)row, crt_s_unit(r.y)), o, d);
+  return r.z;
+}
 
 CRT_DI uint32_t lane_id() { return threadIdx.x & 31u; }
 CRT_DI uint32_t lanemask_lt() {
@@ -349,7 +364,9 @@ CRT_DI bool tail_handoff(const Levels &lv, const uint32_t launch, const bool wan
 // MODE: 2 = this loop.  (0 = while-while and 1 = merged single loop were the round-1 predecessors; their measurements are
 // in profiles/r1_tuning.md, their code is gone.)
 // ------------------------------------------------------------------------------------------------------------
-template <bool PRIMARY, bool COUNT, int REFILL, int MODE, bool CULL, bool WIDE>
+// JITTER (PRIMARY only): level 0 of a GI frame, jittered primary rays (a template flag, so that the unsampled primary
+// kernels keep their register allocation)
+template <bool PRIMARY, bool COUNT, int REFILL, int MODE, bool CULL, bool WIDE, bool JITTER = false>
 __global__ void __launch_bounds__(CRT_TRAV_BLOCK, PRIMARY ? CRT_TRAV_MIN_BLOCKS : CRT_TRAV_MIN_BLOCKS_SEC) k_closest(const DScene sc, const Frame fr, const Levels lv, const uint32_t level,
                                                 uint32_t *__restrict__ work_counter) {
   static_assert(MODE == 2, "only loop mode 2 is implemented");
@@ -393,7 +410,12 @@ __global__ void __launch_bounds__(CRT_TRAV_BLOCK, PRIMARY ? CRT_TRAV_MIN_BLOCKS 
         if (PRIMARY) {
           uint32_t row, col;
           valid = item_pixel(fr, sc, fr.item_begin + i, row, col);
-          if (valid) primary_ray(fr.cam, sc.width, sc.height, row, col, ray.o, ray.d);
+          if (valid) {
+            if (JITTER)
+              jittered_primary_ray(fr, sc.width, sc.height, row, col, ray.o, ray.d);
+            else
+              primary_ray(fr.cam, sc.width, sc.height, row, col, ray.o, ray.d);
+          }
         } else {
           const float4 o = lv.ray_o[node_base - lv.offset[1] + i];
           const float4 d = lv.ray_d[node_base - lv.offset[1] + i];
@@ -525,21 +547,45 @@ CRT_DI V3 texture_color(const DScene &sc, const DTexture &t, const uint4 sh, flo
 // getBarycentricCoordinates (Triangle.cpp:63-73), the set-up halves of calculateReflection / calculateRefraction
 // (RayTracer.cpp:358-417) and Texture::getColor.  Children are compacted into level+1 with one atomic per warp.
 // ------------------------------------------------------------------------------------------------------------
+// The G diffuse children of a diffuse hit (P, shading normal N) of a GI frame, written to queue slots q0 .. q0 + G - 1:
+// origin P + N * mc_bias, direction crt_s_diffuse_dir, path key of slot j, pixel index.  Out of line: the rejection
+// loop's registers stay out of k_shade's allocation.
+static __device__ __noinline__ void spawn_diffuse(const Frame &fr, const Levels &lv, const V3 P, const V3 N, const uint32_t pix,
+                                                  const uint32_t key, const uint32_t q0, const uint32_t G) {
+  const float n3[3] = {N.x, N.y, N.z};
+  const V3 co = vadd(P, vscale(N, fr.mc_bias));
+  for (uint32_t j = 0; j < G; j++) {
+    float dd[3];
+    crt_s_diffuse_dir(fr.seed, fr.frame_index, pix, fr.sample, key, j, n3, dd);
+    lv.ray_o[q0 + j] = make_float4(co.x, co.y, co.z, __uint_as_float(crt_s_child_key(fr.seed, fr.frame_index, pix, fr.sample, key, j)));
+    lv.ray_d[q0 + j] = make_float4(dd[0], dd[1], dd[2], __uint_as_float(pix));
+  }
+}
+
+// GI: frames under the sampling contract (crt_sampling.h): jittered level 0, path keys carried in ray_o.w / pixel index in
+// ray_d.w, and every diffuse hit also spawns G diffuse children (COMB_GI).  GI = false is the unsampled kernel.
+template <bool GI>
 __global__ void __launch_bounds__(256) k_shade(const DScene sc, const Frame fr, const Levels lv, const uint32_t level) {
   const uint32_t total = (level == 0) ? fr.n_items0 : lv.counts[level];
   const uint32_t node_base = lv.offset[level];
   const uint32_t rounded = (total + 31u) & ~31u;
-  uint32_t n_refl = 0, n_refr = 0, n_prim = 0;
+  uint32_t n_refl = 0, n_refr = 0, n_prim = 0, n_diff = 0;
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < rounded; i += gridDim.x * blockDim.x) {
     bool valid = i < total;
     const uint32_t node = node_base + i;
     V3 o = mk(0, 0, 0), d = mk(0, 0, 0);
+    uint32_t key = 0, pix = 0;  // GI: path key of this ray, global pixel index
     if (valid) {
       if (level == 0) {
         uint32_t row, col;
         valid = item_pixel(fr, sc, fr.item_begin + i, row, col);
         if (valid) {
-          primary_ray(fr.cam, sc.width, sc.height, row, col, o, d);
+          if (GI) {
+            key = jittered_primary_ray(fr, sc.width, sc.height, row, col, o, d);
+            pix = row * sc.width + col;
+          } else {
+            primary_ray(fr.cam, sc.width, sc.height, row, col, o, d);
+          }
           n_prim++;
         }
       } else {
@@ -547,6 +593,10 @@ __global__ void __launch_bounds__(256) k_shade(const DScene sc, const Frame fr, 
         const float4 rd = lv.ray_d[node - lv.offset[1]];
         o = mk(ro.x, ro.y, ro.z);
         d = mk(rd.x, rd.y, rd.z);
+        if (GI) {
+          key = __float_as_uint(ro.w);
+          pix = __float_as_uint(rd.w);
+        }
       }
     }
     uint32_t want_children = 0, want_diffuse = 0;
@@ -588,6 +638,10 @@ __global__ void __launch_bounds__(256) k_shade(const DScene sc, const Frame fr, 
         base = (mat.texture != CRT_INVALID)
                    ? texture_color(sc, sc.textures[mat.texture], sh, u, v, fsub(fsub(1.0f, u), v))
                    : mk(mat.albedo[0], mat.albedo[1], mat.albedo[2]);
+        if (GI) {  // G diffuse children; beyond max_depth none is traced and each contributes the background
+          kind = COMB_GI;
+          if (child_traced) want_children = fr.gi_samples;
+        }
       } else if (mat.type == 1u) {  // Reflective: calculateReflection            RayTracer.cpp:366-373
         c0o = vadd(P, vscale(N, fr.reflection_bias));
         c0d = vnorm(vnorm(vreflect(d, N)));  // getNormalized() then shootRay's normalize
@@ -642,15 +696,25 @@ __global__ void __launch_bounds__(256) k_shade(const DScene sc, const Frame fr, 
     const uint32_t child = warp_alloc(&lv.counts[level + 1], want_children);
     const uint32_t dslot = warp_alloc(&lv.counts[CRT_MAX_LEVELS], want_diffuse);
     if (!valid) continue;
-    if (want_children) {
+    if (GI && kind == COMB_GI) {
+      const uint32_t cbase = want_children ? lv.offset[level + 1] + child : CRT_INVALID;
+      if (want_children) spawn_diffuse(fr, lv, P, N, pix, key, cbase - lv.offset[1], want_children);
+      n_diff += want_children;
+      lv.comb[node] = make_uint4(COMB_GI, cbase, dslot, fr.gi_samples);
+      float4 *q = lv.dq + 3 * (size_t)dslot;
+      q[0] = make_float4(P.x, P.y, P.z, __uint_as_float(node));
+      q[1] = make_float4(N.x, N.y, N.z, base.x);
+      q[2] = make_float4(base.y, base.z, 0.f, 0.f);
+    } else if (want_children) {
       const uint32_t cbase = lv.offset[level + 1] + child;
       const uint32_t q = cbase - lv.offset[1];
-      lv.ray_o[q] = make_float4(c0o.x, c0o.y, c0o.z, __uint_as_float(node));
-      lv.ray_d[q] = make_float4(c0d.x, c0d.y, c0d.z, __uint_as_float(2u));
+      // GI: children carry their path key (reflection = slot 0, refraction = slot 1) and the pixel index
+      lv.ray_o[q] = make_float4(c0o.x, c0o.y, c0o.z, __uint_as_float(GI ? crt_s_child_key(fr.seed, fr.frame_index, pix, fr.sample, key, 0u) : node));
+      lv.ray_d[q] = make_float4(c0d.x, c0d.y, c0d.z, __uint_as_float(GI ? pix : 2u));
       n_refl++;
       if (want_children == 2) {
-        lv.ray_o[q + 1] = make_float4(c1o.x, c1o.y, c1o.z, __uint_as_float(node));
-        lv.ray_d[q + 1] = make_float4(c1d.x, c1d.y, c1d.z, __uint_as_float(3u));
+        lv.ray_o[q + 1] = make_float4(c1o.x, c1o.y, c1o.z, __uint_as_float(GI ? crt_s_child_key(fr.seed, fr.frame_index, pix, fr.sample, key, 1u) : node));
+        lv.ray_d[q + 1] = make_float4(c1d.x, c1d.y, c1d.z, __uint_as_float(GI ? pix : 3u));
         n_refr++;
       }
       lv.comb[node] = make_uint4(kind, cbase, kind == COMB_REFLECT ? mat_index : cbase + 1, __float_as_uint(fresnel));
@@ -678,6 +742,12 @@ __global__ void __launch_bounds__(256) k_shade(const DScene sc, const Frame fr, 
     if (a) atomicAdd(&lv.stats[0], a);
     if (b) atomicAdd(&lv.stats[2], b);
     if (c) atomicAdd(&lv.stats[3], c);
+  }
+  if (GI) {
+    unsigned long long g = n_diff;
+#pragma unroll
+    for (int s = 16; s > 0; s >>= 1) g += __shfl_xor_sync(CRT_FULL_MASK, g, s);
+    if (lane_id() == 0 && g) atomicAdd(&lv.stats[41], g);
   }
 }
 
@@ -712,7 +782,9 @@ CRT_DI float shadow_limit(const Ray &ray, const float dist) {
   return dist * 1.0001f + 1e-4f + 1e-6f * (fabsf(ray.o.x) + fabsf(ray.o.y) + fabsf(ray.o.z));
 }
 
-template <int COUNT, int REFILL, int MODE, bool CULL, bool WIDE>
+// SKIPR: shadow rays ignore refractive meshes, as the reference does only when !useGI (AccelerationStructure.cpp:67-71);
+// GI frames instantiate SKIPR = false.
+template <int COUNT, int REFILL, int MODE, bool CULL, bool WIDE, bool SKIPR = true>
 __global__ void __launch_bounds__(CRT_TRAV_BLOCK, CRT_TRAV_MIN_BLOCKS) k_shadow(const DScene sc, const Frame fr, const Levels lv,
                                                                              uint32_t *__restrict__ work_counter) {
   static_assert(MODE == 2, "only loop mode 2 is implemented");
@@ -804,7 +876,7 @@ __global__ void __launch_bounds__(CRT_TRAV_BLOCK, CRT_TRAV_MIN_BLOCKS) k_shadow(
       for (;;) {
         const bool slow = active && tv.tref == tv.tend && tv.cur == tv.cend;
         if (!__any_sync(CRT_FULL_MASK, slow)) break;
-        if (slow && trav_slow<true, (COUNT == 1 ? 0 : (WIDE ? 2 : 1)), CULL>(tv, sc, ray) == TRAV_DONE) {
+        if (slow && trav_slow<SKIPR, (COUNT == 1 ? 0 : (WIDE ? 2 : 1)), CULL>(tv, sc, ray) == TRAV_DONE) {
           lv.vis[slot] = occluded ? 0 : 1;
           active = false;
           CRT_PC_RAY_DONE(1, ray_iters)
@@ -967,7 +1039,8 @@ __global__ void k_mark(uint32_t *flag) {
   if (threadIdx.x == 0) *reinterpret_cast<volatile uint32_t *>(flag) = 1u;
 }
 
-template <bool SHADOW, bool PRIMARY, bool CULL, int GW>
+// SKIPR: shadow rays ignore refractive meshes (false in GI frames, see k_shadow)
+template <bool SHADOW, bool PRIMARY, bool CULL, int GW, bool SKIPR = true>
 __global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_coop(const DScene sc, const Frame fr, const Levels lv, const uint32_t level, const uint32_t early) {
   constexpr uint32_t NG = 32u / GW;            // walks per warp
   constexpr uint32_t CAP = CRT_COOP_CAP / NG;  // LIFO entries per walk
@@ -1039,7 +1112,10 @@ __global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_co
         } else if (PRIMARY) {
           uint32_t row, col;
           item_pixel(fr, sc, fr.item_begin + (id - lv.offset[0]), row, col);  // valid: the main kernel started this ray
-          primary_ray(fr.cam, sc.width, sc.height, row, col, ray.o, ray.d);
+          if (fr.gi)
+            jittered_primary_ray(fr, sc.width, sc.height, row, col, ray.o, ray.d);
+          else
+            primary_ray(fr.cam, sc.width, sc.height, row, col, ray.o, ray.d);
         } else {
           const float4 o = lv.ray_o[id - lv.offset[1]], d = lv.ray_d[id - lv.offset[1]];
           ray.o = mk(o.x, o.y, o.z);
@@ -1109,7 +1185,7 @@ __global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_co
       } else if (mref != mend) {
         const uint32_t m = __ldg(&sc.top_refs[mref++]);
         const DMesh me = sc.meshes[m];
-        bool skip = SHADOW && sc.materials[me.material].type == 3u;  // shadow rays ignore refractive meshes (AccelerationStructure.cpp:67-71)
+        bool skip = SHADOW && SKIPR && sc.materials[me.material].type == 3u;  // shadow rays ignore refractive meshes (AccelerationStructure.cpp:67-71)
         if (sc.dedup_meshes == 1u) {  // (scenes with more than 64 meshes: the rest of a handed-off walk re-walks a mesh for
           const unsigned long long bit = 1ull << (m & 63u);  //  every listing, like the reference; same result)
           skip = skip || (seen & bit) != 0ull;
@@ -1289,6 +1365,9 @@ __global__ void __launch_bounds__(256) k_accumulate(const DScene sc, const Frame
 //   reflective : Color(0,0,0) += albedo (*) R                                    RayTracer.cpp:369-373
 //   refractive : F * R + (1 - F) * T   |   R on total internal reflection       RayTracer.cpp:414, 416
 // ------------------------------------------------------------------------------------------------------------
+//   GI diffuse : (D + base (*) S) / float(G + 1), S = ((0 + L_0) + L_1) + ...,   D = the light sum k_accumulate left in
+//                color[node], base from the diffuse item (sampling contract, DESIGN.md 3.10)
+template <bool GI>
 __global__ void __launch_bounds__(256) k_resolve(const DScene sc, const Frame fr, const Levels lv, const uint32_t level) {
   const uint32_t total = (level == 0) ? fr.n_items0 : lv.counts[level];
   const uint32_t node_base = lv.offset[level];
@@ -1300,6 +1379,18 @@ __global__ void __launch_bounds__(256) k_resolve(const DScene sc, const Frame fr
     }
     const uint4 cb = lv.comb[node];
     if (cb.x == COMB_FINAL) continue;
+    if (GI && cb.x == COMB_GI) {
+      const float4 D = lv.color[node], q1 = lv.dq[3 * (size_t)cb.z + 1], q2 = lv.dq[3 * (size_t)cb.z + 2];
+      V3 S = mk(0.f, 0.f, 0.f);
+      for (uint32_t j = 0; j < cb.w; j++) {
+        const float4 L = cb.y != CRT_INVALID ? lv.color[cb.y + j] : make_float4(sc.bg[0], sc.bg[1], sc.bg[2], 0.f);
+        S = vadd(S, mk(L.x, L.y, L.z));
+      }
+      const float g1 = (float)(cb.w + 1u);
+      lv.color[node] = make_float4(fdiv(fadd(D.x, fmul(q1.w, S.x)), g1), fdiv(fadd(D.y, fmul(q2.x, S.y)), g1),
+                                   fdiv(fadd(D.z, fmul(q2.y, S.z)), g1), 0.f);
+      continue;
+    }
     const float4 A = lv.color[cb.y];
     V3 out;
     if (cb.x == COMB_REFLECT) {
@@ -1313,6 +1404,34 @@ __global__ void __launch_bounds__(256) k_resolve(const DScene sc, const Frame fr
       out = mk(A.x, A.y, A.z);
     }
     lv.color[node] = make_float4(out.x, out.y, out.z, 0.f);
+  }
+}
+
+// Sample pass fr.sample of a GI frame: acc = acc + c_s in sample order (acc starts at (0,0,0)); the last pass leaves
+// acc / float(spp) in the level-0 colour, and sample 0's primary hit in the level-0 hit record, for k_store.  Counts
+// the shadow rays of every pass but the last (k_store counts those of the last).
+__global__ void __launch_bounds__(256) k_sample_acc(const DScene sc, const Frame fr, const Levels lv, float4 *__restrict__ acc,
+                                                    uint2 *__restrict__ hit0) {
+  if (blockIdx.x == 0 && threadIdx.x == 0 && fr.sample + 1u < fr.spp)
+    atomicAdd(&lv.stats[1], (unsigned long long)lv.counts[CRT_MAX_LEVELS] * sc.n_lights);
+  const bool last = fr.sample + 1u == fr.spp;
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x) {
+    const uint32_t node = lv.offset[0] + i;
+    const float4 c = lv.color[node];
+    const float4 a0 = fr.sample == 0 ? make_float4(0.f, 0.f, 0.f, 0.f) : acc[i];
+    const V3 a = vadd(mk(a0.x, a0.y, a0.z), mk(c.x, c.y, c.z));
+    if (fr.sample == 0 && !last) hit0[i] = make_uint2(lv.hit_tri[node], __float_as_uint(lv.hit_t[node]));
+    if (last) {
+      const float n = (float)fr.spp;
+      lv.color[node] = make_float4(fdiv(a.x, n), fdiv(a.y, n), fdiv(a.z, n), 0.f);
+      if (fr.sample != 0) {
+        const uint2 h = hit0[i];
+        lv.hit_tri[node] = h.x;
+        lv.hit_t[node] = __uint_as_float(h.y);
+      }
+    } else {
+      acc[i] = make_float4(a.x, a.y, a.z, 0.f);
+    }
   }
 }
 

@@ -197,6 +197,8 @@ struct crtb200_ctx {
     DevBuf<uint4> comb;
     DevBuf<uint8_t> vis;
     DevBuf<uint4> ovf;          // walks handed off to k_coop (3 x uint4 per record)
+    DevBuf<float4> acc;         // GI frames: per level-0 item of the chunk, the running sample sum (k_sample_acc)
+    DevBuf<uint2> hit0;         //            ... and sample 0's primary hit
     uint32_t *work = nullptr;   // into ctl
     cudaStream_t stream = nullptr;
     cudaEvent_t done = nullptr;
@@ -205,7 +207,7 @@ struct crtb200_ctx {
     cudaEvent_t coop_fork = nullptr, coop_join = nullptr;
     void release() {
       ray_o.release(); ray_d.release(); color.release(); dq.release(); hit_tri.release(); ctl.release();
-      hit_t.release(); comb.release(); vis.release(); ovf.release();
+      hit_t.release(); comb.release(); vis.release(); ovf.release(); acc.release(); hit0.release();
     }
   };
   std::vector<QueueSet> sets;
@@ -231,6 +233,12 @@ struct crtb200_ctx {
   int blocks_closest = 0, blocks_closest_sec = 0, blocks_shadow = 0, blocks_coop = 0;
   crtb200_stats last{};
   bool last_pending = false;
+  // sampling contract (crtb200_set_sampling); sampling.use_gi = 0: unsampled frames
+  crtb200_sampling sampling{};
+  uint32_t frame_offset = 0;  // crtb200_render_frames: added to sampling.frame_index for frame f
+  uint64_t last_diffuse = 0;  // diffuse rays of the last render (stats[41])
+  uint32_t last_samples = 1;
+  uint32_t cap_branch = 0;    // worst-case children per ray-tree node the queues were planned for
 
   // multi-GPU (crtb200_create_multi): this context is the primary (device_ids[0]).  A frame's 8x4-pixel tiles are dealt
   // round-robin over primary + peers (scene replicated); every GPU's k_store writes its pixels STRAIGHT into the
@@ -417,6 +425,33 @@ int crtb200_set_concurrency(crtb200_ctx *c, uint32_t chunks_in_flight) {
   c->concurrency = chunks_in_flight;
   c->cap_items = 0;
   for (crtb200_ctx *p : c->peers) crtb200_set_concurrency(p, chunks_in_flight);
+  return CRTB200_OK;
+}
+
+int crtb200_set_sampling(crtb200_ctx *c, const crtb200_sampling *s) {
+  ErrScope scope(c);
+  if (!c) return fail(CRTB200_ERR_ARG, "ctx is null");
+  crtb200_sampling v{};
+  if (s && s->use_gi) {
+    if (s->rays_per_pixel == 0) return fail(CRTB200_ERR_ARG, "rays_per_pixel must be at least 1 with GI on");
+    if (s->gi_samples > 1024) return fail(CRTB200_ERR_ARG, "gi_samples must be at most 1024");
+    v = *s;
+    v.use_gi = 1;
+  }
+  c->sampling = v;
+  for (crtb200_ctx *p : c->peers) crtb200_set_sampling(p, &v);
+  return CRTB200_OK;
+}
+
+int crtb200_last_sampling_stats(crtb200_ctx *c, crtb200_sampling_stats *stats) {
+  ErrScope scope(c);
+  if (!c || !stats) return fail(CRTB200_ERR_ARG, "null argument");
+  crtb200_stats unused;
+  const int rc = crtb200_last_stats(c, &unused);  // synchronises a pending render_device frame
+  if (rc) return rc;
+  stats->rays_diffuse = c->last_diffuse;
+  stats->samples = c->last_samples;
+  stats->reserved = 0;
   return CRTB200_OK;
 }
 
@@ -808,21 +843,22 @@ static int upload_one(crtb200_ctx *c, const crtb200_scene *s) {
 }
 
 // ---- frame planning ------------------------------------------------------------------------------------------
+// worst-case children of one ray-tree node: refractive hits spawn two (RayTracer.cpp:398-412), reflective ones one, and
+// in GI frames diffuse hits G (crtb200_sampling.gi_samples)
+static uint32_t node_branching(const crtb200_ctx *c) {
+  uint32_t b = c->has_refractive ? 2u : (c->has_reflective ? 1u : 0u);
+  if (c->sampling.use_gi) b = std::max(b, c->sampling.gi_samples);
+  return b;
+}
+
 static uint32_t branching_sum(const crtb200_ctx *c, uint32_t max_depth, uint64_t *per_level) {
-  // worst-case rays per level-0 item at each level (refractive hits spawn two children, RayTracer.cpp:398-412)
-  uint64_t sum = 0;
+  // worst-case rays per level-0 item at each level: branching^level, saturated at 2^40 (far beyond any queue budget)
+  const uint64_t branch = node_branching(c), cap = 1ull << 40;
+  uint64_t sum = 0, b = 1;
   for (uint32_t l = 0; l <= max_depth; l++) {
-    uint64_t b = 1;
-    if (l > 0) {
-      if (c->has_refractive)
-        b = 1ull << std::min<uint32_t>(l, 40);
-      else if (c->has_reflective)
-        b = 1;
-      else
-        b = 0;
-    }
     per_level[l] = b;
     sum += b;
+    b = std::min<uint64_t>(b * branch, cap);
   }
   return (uint32_t)std::min<uint64_t>(sum, 0xFFFFFFFFull);
 }
@@ -861,7 +897,10 @@ static int plan_queues(crtb200_ctx *c, uint32_t shard_items, uint32_t max_depth,
   }
   uint64_t items = c->queue_budget / (bytes_per_node * sum * n_sets);
   items &= ~31ull;
-  if (items < 32 * 64) return fail(CRTB200_ERR_MEMORY, "queue budget too small for one chunk at this ray depth");
+  if (items < 32 * 64)
+    return fail(CRTB200_ERR_MEMORY, c->sampling.use_gi ? "queue budget too small for one chunk of 2048 pixels: the GI ray tree has up to "
+                                                             "gi_samples^max_depth nodes per pixel; lower gi_samples or max_depth"
+                                                       : "queue budget too small for one chunk at this ray depth");
   // host-bound frames: one chunk per stream at 1080p, two at 4K (a band's copy overlaps the traversal of the next band;
   // every chunk pays its own kernel tails and, in reflective scenes, the latency of every level again)
   uint32_t per_set = (pipelined && n_sets > 1 && shard_items >= (1u << 22)) ? 2u : 1u;
@@ -875,7 +914,7 @@ static int plan_queues(crtb200_ctx *c, uint32_t shard_items, uint32_t max_depth,
   if (items < 32) return fail(CRTB200_ERR_MEMORY, "too many lights x ray-tree nodes for 32-bit queue slots");
   if (items >= row_items) items = (items / row_items) * row_items;  // whole tile rows (band copies need it)
   c->n_chunks = (uint32_t)((shard_items + items - 1) / items);
-  if (c->cap_items == items && c->cap_depth == max_depth && c->cap_sets == n_sets) return CRTB200_OK;
+  if (c->cap_items == items && c->cap_depth == max_depth && c->cap_sets == n_sets && c->cap_branch == node_branching(c)) return CRTB200_OK;
   if (c->sets.size() < n_sets) c->sets.resize(n_sets);
   if (!c->fork_ev) CUDA_TRY(cudaEventCreateWithFlags(&c->fork_ev, cudaEventDisableTiming));
   for (uint32_t k = 0; k < n_sets; k++) {
@@ -936,6 +975,7 @@ static int plan_queues(crtb200_ctx *c, uint32_t shard_items, uint32_t max_depth,
   c->cap_items = (uint32_t)items;
   c->cap_depth = max_depth;
   c->cap_sets = n_sets;
+  c->cap_branch = node_branching(c);
   return CRTB200_OK;
 }
 
@@ -982,7 +1022,9 @@ static size_t dyn_smem(const crtb200_ctx *c, int block) { return (size_t)c->sc.d
 template <bool COUNT, bool CULL, bool WIDE>
 static void launch_closest_w(crtb200_ctx *c, bool primary, const Frame &fr, const Levels &lv, uint32_t level, uint32_t *work,
                              cudaStream_t st) {
-  if (primary)
+  if (primary && fr.gi)
+    k_closest<true, COUNT, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, CULL, WIDE, true><<<c->blocks_closest, CRT_TRAV_BLOCK, dyn_smem(c, CRT_TRAV_BLOCK), st>>>(c->sc, fr, lv, level, work);
+  else if (primary)
     k_closest<true, COUNT, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, CULL, WIDE><<<c->blocks_closest, CRT_TRAV_BLOCK, dyn_smem(c, CRT_TRAV_BLOCK), st>>>(c->sc, fr, lv, level, work);
   else
     k_closest<false, COUNT, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, CULL, WIDE><<<c->blocks_closest_sec, CRT_TRAV_BLOCK, dyn_smem(c, CRT_TRAV_BLOCK), st>>>(c->sc, fr, lv, level, work);
@@ -997,12 +1039,27 @@ static void launch_closest(crtb200_ctx *c, bool primary, const Frame &fr, const 
   else
     launch_closest_w<COUNT, CULL, false>(c, primary, fr, lv, level, work, st);
 }
-template <int COUNT, bool CULL>
+template <int COUNT, bool CULL, bool SKIPR = true>
 static void launch_shadow(crtb200_ctx *c, const Frame &fr, const Levels &lv, uint32_t *work, cudaStream_t st) {
   if (COUNT != 1 && c->sc.dedup_meshes == 2u)
-    k_shadow<COUNT, CRT_REFILL_SHADOW, CRT_LOOP_MODE, CULL, (COUNT != 1)><<<c->blocks_shadow, CRT_TRAV_BLOCK, dyn_smem(c, CRT_TRAV_BLOCK), st>>>(c->sc, fr, lv, work);
+    k_shadow<COUNT, CRT_REFILL_SHADOW, CRT_LOOP_MODE, CULL, (COUNT != 1), SKIPR><<<c->blocks_shadow, CRT_TRAV_BLOCK, dyn_smem(c, CRT_TRAV_BLOCK), st>>>(c->sc, fr, lv, work);
   else
-    k_shadow<COUNT, CRT_REFILL_SHADOW, CRT_LOOP_MODE, CULL, false><<<c->blocks_shadow, CRT_TRAV_BLOCK, 0, st>>>(c->sc, fr, lv, work);
+    k_shadow<COUNT, CRT_REFILL_SHADOW, CRT_LOOP_MODE, CULL, false, SKIPR><<<c->blocks_shadow, CRT_TRAV_BLOCK, 0, st>>>(c->sc, fr, lv, work);
+}
+// the shadow pass of one chunk in the flavour the options ask for; SKIPR = false in GI frames
+template <bool SKIPR>
+static void launch_shadow_pass(crtb200_ctx *c, const crtb200_options *o, bool cull, const Frame &fr, const Levels &lv, uint32_t *work,
+                               cudaStream_t st) {
+  if (o->count_work == 1)
+    launch_shadow<1, false, SKIPR>(c, fr, lv, work, st);
+  else if (o->count_work == 2 && cull)
+    launch_shadow<2, true, SKIPR>(c, fr, lv, work, st);
+  else if (o->count_work == 2)
+    launch_shadow<2, false, SKIPR>(c, fr, lv, work, st);
+  else if (cull)
+    launch_shadow<0, true, SKIPR>(c, fr, lv, work, st);
+  else
+    launch_shadow<0, false, SKIPR>(c, fr, lv, work, st);
 }
 
 // k_coop around one traversal launch (DESIGN.md 3.8).  coop_begin forks the side stream BEFORE the traversal kernel is
@@ -1017,12 +1074,12 @@ static int coop_begin(crtb200_ctx *c, crtb200_ctx::QueueSet &q, bool secondary_l
   CUDA_TRY(cudaStreamWaitEvent(q.coop_stream, q.coop_fork, 0));
   return CRTB200_OK;
 }
-template <bool SHADOW, bool CULL>
+template <bool SHADOW, bool CULL, bool SKIPR = true>
 static int coop_end(crtb200_ctx *c, crtb200_ctx::QueueSet &q, bool primary, const Frame &fr, uint32_t level, uint32_t &launches) {
   const uint32_t launch = SHADOW ? (uint32_t)CRT_MAX_LEVELS : level;
   auto run = [&](int blocks, cudaStream_t st, uint32_t early) {
     if (SHADOW)
-      k_coop<true, false, CULL, CRT_COOP_GROUP><<<blocks, 32 * CRT_COOP_WARPS, 0, st>>>(c->sc, fr, q.lv, 0, early);
+      k_coop<true, false, CULL, CRT_COOP_GROUP, SKIPR><<<blocks, 32 * CRT_COOP_WARPS, 0, st>>>(c->sc, fr, q.lv, 0, early);
     else if (primary)
       k_coop<false, true, CULL, CRT_COOP_GROUP><<<blocks, 32 * CRT_COOP_WARPS, 0, st>>>(c->sc, fr, q.lv, level, early);
     else
@@ -1075,18 +1132,27 @@ static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb20
   fr.shard_count = shard_count;
   fr.mask = c->mask_needed ? c->mask.p : nullptr;
   fr.max_depth = o->max_depth;
-  fr.resolve = (c->has_reflective || c->has_refractive) ? 1u : 0u;
+  // GI frames (sampling contract, DESIGN.md 3.10): spp sample-major passes per chunk, each the whole level loop below
+  const bool gi = c->sampling.use_gi != 0;
+  fr.resolve = (c->has_reflective || c->has_refractive || gi) ? 1u : 0u;
   fr.shadow_bias = o->shadow_bias;
   fr.reflection_bias = o->reflection_bias;
   fr.refraction_bias = o->refraction_bias;
+  fr.gi = gi ? 1u : 0u;
+  fr.gi_samples = gi ? c->sampling.gi_samples : 0u;
+  fr.spp = gi ? c->sampling.rays_per_pixel : 1u;
+  fr.seed = c->sampling.seed;
+  fr.frame_index = c->sampling.frame_index + c->frame_offset;
+  fr.mc_bias = c->sampling.monte_carlo_bias;
   const uint32_t shard_tiles = (fr.n_tiles > o->shard_index) ? (fr.n_tiles - o->shard_index + shard_count - 1) / shard_count : 0;
   const uint32_t shard_items = shard_tiles * 32u;
   // unsharded frames: chunks are whole rows of tiles, so a chunk owns a contiguous band of image rows
   const uint32_t row_items = (shard_count == 1) ? fr.tiles_x * 32u : 32u;
   rc = plan_queues(c, std::max(shard_items, 32u), o->max_depth, row_items, host != nullptr);
   if (rc) return rc;
-  const bool secondary = c->has_reflective || c->has_refractive;
+  const bool secondary = c->has_reflective || c->has_refractive || gi;
   const uint32_t levels = secondary ? o->max_depth + 1 : 1;
+  c->last_samples = fr.spp;
   // Band copies need chunks that own whole rows of tiles: with a small queue budget or a deep refractive scene a chunk
   // is smaller than a tile row, two chunks on different streams would then share a 4-row band and a band copy could
   // pick up the other chunk's stale pixels.  Then the caller copies the whole frame after the join instead.
@@ -1126,76 +1192,91 @@ static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb20
     cudaStream_t qs = q.stream;
     fr.item_begin = begin;
     fr.n_items0 = std::min(c->cap_items, shard_items - begin);
-    CUDA_TRY(cudaMemsetAsync(q.ctl.p, 0, q.ctl.n * sizeof(uint32_t), qs));
-    q.lv.tail_iters = handoff ? (uint32_t)(c->tail_iters + 1) : 0u;
-    q.lv.skip_zero_terms = (o->traversal == 0 && o->count_work != 1) ? 1u : 0u;
-    q.lv.tail_start = (uint32_t)c->tail_start;
-    q.lv.tail_start_closest = (uint32_t)c->tail_start_closest;
-    q.lv.tail_small = (uint32_t)c->tail_small;
-    for (uint32_t l = 0; l < levels; l++) {
+    if (gi) {
+      CUDA_TRY(q.acc.ensure(c->cap_items));
+      CUDA_TRY(q.hit0.ensure(c->cap_items));
+    }
+    for (uint32_t s = 0; s < fr.spp; s++) {
+      fr.sample = s;
+      CUDA_TRY(cudaMemsetAsync(q.ctl.p, 0, q.ctl.n * sizeof(uint32_t), qs));
+      q.lv.tail_iters = handoff ? (uint32_t)(c->tail_iters + 1) : 0u;
+      q.lv.skip_zero_terms = (o->traversal == 0 && o->count_work != 1) ? 1u : 0u;
+      q.lv.tail_start = (uint32_t)c->tail_start;
+      q.lv.tail_start_closest = (uint32_t)c->tail_start_closest;
+      q.lv.tail_small = (uint32_t)c->tail_small;
+      for (uint32_t l = 0; l < levels; l++) {
+        if (per_kernel) {
+          cudaEventRecord(next_event(c), qs);
+          c->kev_kind.push_back(0);
+        }
+        if (handoff) {
+          rc = coop_begin(c, q, l != 0);
+          if (rc) return rc;
+        }
+        if (o->count_work && cull)
+          launch_closest<true, true>(c, l == 0, fr, q.lv, l, q.work + CRT_CTL_STRIDE * l, qs);
+        else if (o->count_work)
+          launch_closest<true, false>(c, l == 0, fr, q.lv, l, q.work + CRT_CTL_STRIDE * l, qs);
+        else if (cull)
+          launch_closest<false, true>(c, l == 0, fr, q.lv, l, q.work + CRT_CTL_STRIDE * l, qs);
+        else
+          launch_closest<false, false>(c, l == 0, fr, q.lv, l, q.work + CRT_CTL_STRIDE * l, qs);
+        if (handoff) {
+          if (per_kernel) {
+            cudaEventRecord(next_event(c), qs);
+            cudaEventRecord(next_event(c), qs);
+            c->kev_kind.push_back(2);
+          }
+          rc = cull ? coop_end<false, true>(c, q, l == 0, fr, l, launches) : coop_end<false, false>(c, q, l == 0, fr, l, launches);
+          if (rc) return rc;
+        }
+        if (per_kernel) cudaEventRecord(next_event(c), qs);
+        if (gi)
+          k_shade<true><<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, l);
+        else
+          k_shade<false><<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, l);
+        launches += 2;
+      }
       if (per_kernel) {
         cudaEventRecord(next_event(c), qs);
-        c->kev_kind.push_back(0);
+        c->kev_kind.push_back(1);
       }
+      uint32_t *swork = q.work + CRT_CTL_STRIDE * CRT_MAX_LEVELS;
       if (handoff) {
-        rc = coop_begin(c, q, l != 0);
+        rc = coop_begin(c, q, false);
         if (rc) return rc;
       }
-      if (o->count_work && cull)
-        launch_closest<true, true>(c, l == 0, fr, q.lv, l, q.work + CRT_CTL_STRIDE * l, qs);
-      else if (o->count_work)
-        launch_closest<true, false>(c, l == 0, fr, q.lv, l, q.work + CRT_CTL_STRIDE * l, qs);
-      else if (cull)
-        launch_closest<false, true>(c, l == 0, fr, q.lv, l, q.work + CRT_CTL_STRIDE * l, qs);
+      if (gi)
+        launch_shadow_pass<false>(c, o, cull, fr, q.lv, swork, qs);
       else
-        launch_closest<false, false>(c, l == 0, fr, q.lv, l, q.work + CRT_CTL_STRIDE * l, qs);
+        launch_shadow_pass<true>(c, o, cull, fr, q.lv, swork, qs);
       if (handoff) {
         if (per_kernel) {
           cudaEventRecord(next_event(c), qs);
           cudaEventRecord(next_event(c), qs);
-          c->kev_kind.push_back(2);
+          c->kev_kind.push_back(3);
         }
-        rc = cull ? coop_end<false, true>(c, q, l == 0, fr, l, launches) : coop_end<false, false>(c, q, l == 0, fr, l, launches);
+        if (gi)
+          rc = cull ? coop_end<true, true, false>(c, q, false, fr, 0, launches) : coop_end<true, false, false>(c, q, false, fr, 0, launches);
+        else
+          rc = cull ? coop_end<true, true>(c, q, false, fr, 0, launches) : coop_end<true, false>(c, q, false, fr, 0, launches);
         if (rc) return rc;
       }
       if (per_kernel) cudaEventRecord(next_event(c), qs);
-      k_shade<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, l);
+      k_accumulate<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv);
       launches += 2;
-    }
-    if (per_kernel) {
-      cudaEventRecord(next_event(c), qs);
-      c->kev_kind.push_back(1);
-    }
-    uint32_t *swork = q.work + CRT_CTL_STRIDE * CRT_MAX_LEVELS;
-    if (handoff) {
-      rc = coop_begin(c, q, false);
-      if (rc) return rc;
-    }
-    if (o->count_work == 1)
-      launch_shadow<1, false>(c, fr, q.lv, swork, qs);
-    else if (o->count_work == 2 && cull)
-      launch_shadow<2, true>(c, fr, q.lv, swork, qs);
-    else if (o->count_work == 2)
-      launch_shadow<2, false>(c, fr, q.lv, swork, qs);
-    else if (cull)
-      launch_shadow<0, true>(c, fr, q.lv, swork, qs);
-    else
-      launch_shadow<0, false>(c, fr, q.lv, swork, qs);
-    if (handoff) {
-      if (per_kernel) {
-        cudaEventRecord(next_event(c), qs);
-        cudaEventRecord(next_event(c), qs);
-        c->kev_kind.push_back(3);
+      // (GI frames resolve the last level too: its diffuse hits combine D with G background children)
+      for (uint32_t l = gi ? levels : levels - 1; l-- > 0;) {
+        if (gi)
+          k_resolve<true><<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, l);
+        else
+          k_resolve<false><<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, l);
+        launches++;
       }
-      rc = cull ? coop_end<true, true>(c, q, false, fr, 0, launches) : coop_end<true, false>(c, q, false, fr, 0, launches);
-      if (rc) return rc;
-    }
-    if (per_kernel) cudaEventRecord(next_event(c), qs);
-    k_accumulate<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv);
-    launches += 2;
-    for (uint32_t l = levels - 1; l-- > 0;) {
-      k_resolve<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, l);
-      launches++;
+      if (gi) {
+        k_sample_acc<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, q.acc.p, q.hit0.p);
+        launches++;
+      }
     }
     k_store<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, d_rgb, d_rgb8, d_hits, d_slab);
     launches++;
@@ -1299,6 +1380,7 @@ static int collect_stats(crtb200_ctx *c, bool timed) {
     c->last.handoff_shadow += p->last.handoff_shadow;
     c->last.shadow_rays_zero_term += p->last.shadow_rays_zero_term;
     c->last.kernel_launches += p->last.kernel_launches;
+    c->last_diffuse += p->last_diffuse;
   }
   CUDA_TRY(cudaSetDevice(c->device));
   return CRTB200_OK;
@@ -1362,6 +1444,7 @@ static int collect_stats_one(crtb200_ctx *c, bool timed) {
   c->last.handoff_closest = st[32];
   c->last.handoff_shadow = st[33];
   c->last.shadow_rays_zero_term = st[40];
+  c->last_diffuse = st[41];
 #if CRT_COOP_STATS
   fprintf(stderr, "[coop stats] closest: %llu walks, %llu iterations, %llu box tests, %llu triangle tests | shadow: %llu walks, %llu iterations, %llu box tests, %llu triangle tests\n",
           st[32], st[34], st[35], st[36], st[33], st[37], st[38], st[39]);
@@ -1460,6 +1543,12 @@ static void add_stats(crtb200_stats &total, const crtb200_stats &s) {
   total.levels = s.levels;
 }
 
+// GI frames of a batch: frame f takes Philox key word frame_index + f (on every GPU of a multi-GPU context)
+static void set_frame_offset(crtb200_ctx *c, uint32_t f) {
+  c->frame_offset = f;
+  for (crtb200_ctx *p : c->peers) p->frame_offset = f;
+}
+
 // The animation loop of app/animation.cpp:24-38 (setCamera + render per frame), batched and pipelined: no host
 // synchronisation between frames, two frames in flight -- frame f + 1 is rendered while frame f's pixels travel to the
 // host on a copy stream.  Rectangle lists that leave pixels uncovered need colorBuffer persistence from frame to frame
@@ -1476,13 +1565,18 @@ int crtb200_render_frames(crtb200_ctx *c, const crtb200_camera *cams, uint32_t n
   if (rc) return rc;
   if (c->mask_needed || o->shard_count > 1 || o->count_work != 0 || n_frames < 2) {
     crtb200_stats total{};
+    uint64_t diffuse = 0;
     for (uint32_t f = 0; f < n_frames; f++) {
       crtb200_stats s{};
+      set_frame_offset(c, f);
       rc = crtb200_render(c, cams + f, o, rgb_out ? rgb_out + f * px * 3 : nullptr, rgb8_out ? rgb8_out + f * px * 3 : nullptr, nullptr, &s);
+      set_frame_offset(c, 0);
       if (rc) return rc;
       add_stats(total, s);
+      diffuse += c->last_diffuse;
     }
     total.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    c->last_diffuse = diffuse;
     if (stats) *stats = total;
     return CRTB200_OK;
   }
@@ -1500,7 +1594,9 @@ int crtb200_render_frames(crtb200_ctx *c, const crtb200_camera *cams, uint32_t n
     float *d_rgb = k ? c->frame_b.p : c->frame.p;
     uint8_t *d_rgb8 = rgb8_out ? (k ? c->frame8_b.p : c->frame8.p) : nullptr;
     if (f >= 2) CUDA_TRY(cudaStreamWaitEvent(c->stream, c->copied[k], 0));  // this pair's previous frame has left the device
+    set_frame_offset(c, f);
     rc = enqueue_any(c, cams + f, o, d_rgb, d_rgb8, nullptr, nullptr, c->stream, true, nullptr, nullptr, f > 0);
+    set_frame_offset(c, 0);
     if (rc) return rc;
     launches += c->last.kernel_launches;
     CUDA_TRY(cudaEventRecord(c->rendered[k], c->stream));

@@ -203,4 +203,18 @@ int crtfe_tracer_render(crtfe_tracer *t, const char *path, uint32_t mode, uint32
     if (stats) *stats = t->tracer->lastStats();
   })
 }
+int crtfe_tracer_render_sampled(crtfe_tracer *t, const char *path, uint32_t mode, uint32_t maxDepth, uint32_t literalWalk,
+                                uint32_t useGI, uint32_t giSamples, uint32_t raysPerPixel, float monteCarloBias, uint32_t seed,
+                                float *rgbOut, crtb200_stats *stats) {
+  if (!t) return fail("null argument");
+  CRTFE_TRY({
+    RenderOptions ro(static_cast<RenderOptimization>(mode), maxDepth, useGI != 0, giSamples, raysPerPixel);
+    ro.MONTE_CARLO_BIAS = monteCarloBias;
+    ro.LITERAL_WALK = literalWalk != 0;
+    ro.SEED = seed;
+    const std::vector<float> &buf = t->tracer->renderFlat(path ? path : "", ro);
+    if (rgbOut) std::memcpy(rgbOut, buf.data(), buf.size() * sizeof(float));
+    if (stats) *stats = t->tracer->lastStats();
+  })
+}
 }

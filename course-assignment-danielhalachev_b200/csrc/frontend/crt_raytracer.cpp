@@ -112,7 +112,6 @@ RayTracer::~RayTracer() {
 }
 
 const std::vector<float> &RayTracer::renderFlat(const std::string &pathToImage, RenderOptions ro) {
-  if (ro.USE_GI) throw std::runtime_error("RayTracer::render: USE_GI is not supported by the B200 core");
   // The brute-force and single-AABB modes do not go through the KD trees in the reference: they use the linear scan of
   // RayTracer::trace / hasIntersection (RayTracer.cpp:459-505, 521-537), which breaks equal-t ties by scene order and
   // starts from minDistance = FLT_MAX (so NaN / inf candidates never win) -- not the tree modes' rules.  The B200 core
@@ -143,6 +142,15 @@ const std::vector<float> &RayTracer::renderFlat(const std::string &pathToImage, 
   opt.n_rects = static_cast<uint32_t>(rects.size());
   opt.rects = rects.data();
   opt.traversal = ro.LITERAL_WALK ? 1u : 0u;
+  // RenderOptions' GI members apply to this render only: the context's sampling state follows them on every call
+  crtb200_sampling smp{};
+  smp.use_gi = ro.USE_GI ? 1u : 0u;
+  smp.gi_samples = ro.GI_SAMPLE_SIZE;
+  smp.rays_per_pixel = ro.RAYS_PER_PIXEL;
+  smp.monte_carlo_bias = ro.MONTE_CARLO_BIAS;
+  smp.seed = ro.SEED;
+  if (crtb200_set_sampling(ctx, &smp) != CRTB200_OK)
+    throw std::runtime_error(std::string("crtb200_set_sampling: ") + crtb200_last_error_ctx(ctx));
   if (crtb200_render(ctx, &cam, &opt, colorBuffer.data(), nullptr, nullptr, &stats) != CRTB200_OK)
     throw std::runtime_error(std::string("crtb200_render: ") + crtb200_last_error_ctx(ctx));
   if (!pathToImage.empty()) writePPM(pathToImage, colorBuffer.data(), W, H);

@@ -32,7 +32,7 @@ enum RenderOptimization {
 
 struct RenderOptions {  // RayTracer.h:25-50
   RenderOptimization optimization = B200Wavefront;
-  bool USE_GI = false;  // must stay false: the GI branch is out of scope (clock-seeded RNG, SURVEY 2 #12)
+  bool USE_GI = false;  // GI + jittered supersampling under the reproducible sampling contract (crtb200_set_sampling)
   unsigned MAX_DEPTH = 5;
   unsigned GI_SAMPLE_SIZE = 2;
   unsigned RAYS_PER_PIXEL = 1;
@@ -41,6 +41,7 @@ struct RenderOptions {  // RayTracer.h:25-50
   float REFRACTION_BIAS = 1e-4;
   float MONTE_CARLO_BIAS = 1e-4;
   bool LITERAL_WALK = false;  // extension: crtb200_options::traversal = 1, the visit-all itinerary with nothing skipped (same results)
+  unsigned SEED = 0;          // extension: Philox key of the GI / supersampling random numbers (crtb200_sampling::seed)
   explicit RenderOptions(RenderOptimization optimization = B200Wavefront, unsigned maxDepth = 5, bool useGI = false,
                          unsigned sampleSize = 2, unsigned raysPerPixel = 1, float shadowBias = 1e-4,
                          float reflectionBias = 1e-4, float refractionBias = 1e-4, float monteCarloBias = 1e-4)

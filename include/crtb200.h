@@ -43,7 +43,7 @@ enum { CRTB200_MAT_DIFFUSE = 0, CRTB200_MAT_REFLECTIVE = 1, CRTB200_MAT_CONSTANT
 /* texture classes of include/tracer/Texture.h:18-59 */
 enum { CRTB200_TEX_ALBEDO = 0, CRTB200_TEX_EDGES = 1, CRTB200_TEX_CHECKER = 2, CRTB200_TEX_BITMAP = 3 };
 /* enum RayType { PrimaryRay, ShadowRay, ReflectionRay, RefractionRay, DiffuseRay }  include/tracer/Ray.h:14 */
-enum { CRTB200_RAY_PRIMARY = 0, CRTB200_RAY_SHADOW = 1, CRTB200_RAY_REFLECTION = 2, CRTB200_RAY_REFRACTION = 3 };
+enum { CRTB200_RAY_PRIMARY = 0, CRTB200_RAY_SHADOW = 1, CRTB200_RAY_REFLECTION = 2, CRTB200_RAY_REFRACTION = 3, CRTB200_RAY_DIFFUSE = 4 };
 
 /* One KD-tree node in the REFERENCE's numbering: KDTree<T>::TreeNode (include/tree/KDTree.h:16-21), nodes appended
  * in DFS pre-order by createNode (KDTree.h:33-38), root = 0 of its tree.  A node is a leaf iff leaf_count > 0
@@ -145,7 +145,7 @@ typedef struct crtb200_rect {
   uint32_t row, col, width, height;
 } crtb200_rect;
 
-/* RenderOptions (RayTracer.h:25-50) minus the GI members (out of scope: clock-seeded RNG) + the rectangle list
+/* RenderOptions (RayTracer.h:25-50) minus the GI members (crtb200_sampling, set per context) + the rectangle list
  * the reference's schedulers would produce (RayTracer.cpp:114-202).  n_rects = 0 renders the whole image. */
 typedef struct crtb200_options {
   uint32_t max_depth;    /* MAX_DEPTH, default 5           */
@@ -224,6 +224,35 @@ int crtb200_set_queue_budget(crtb200_ctx *ctx, uint64_t bytes);
 /* chunks of a frame rendered concurrently on separate streams (default 2; 1 = strictly sequential kernels, which is
  * what the per-kernel timers closest_ms / shadow_ms of crtb200_stats require -- they read 0 otherwise) */
 int crtb200_set_concurrency(crtb200_ctx *ctx, uint32_t chunks_in_flight);
+
+/* The GI members of RenderOptions (RayTracer.h:25-50: USE_GI, GI_SAMPLE_SIZE, RAYS_PER_PIXEL, MONTE_CARLO_BIAS) and the
+ * GI / supersampling branch of RayTracer::render and shootRay (RayTracer.cpp:90-104, 331-354; Vector.cpp:124-135), under
+ * this project's reproducible sampling contract (DESIGN.md 3.10) instead of the reference's clock()-seeded rand():
+ * Philox4x32-10 keyed by {seed, frame_index}, counters derived from the global pixel, the sample and the ray's place in
+ * the ray tree, so a frame does not depend on chunking, tile shards or GPU count.  With use_gi = 0 every render call
+ * renders exactly what it renders without this call (rays_per_pixel only matters with GI on, as in the reference). */
+typedef struct crtb200_sampling {
+  uint32_t use_gi;         /* USE_GI                                                                       */
+  uint32_t gi_samples;     /* GI_SAMPLE_SIZE: diffuse bounce rays per diffuse hit (G), at most 1024         */
+  uint32_t rays_per_pixel; /* RAYS_PER_PIXEL: jittered primary rays per pixel, averaged in sample order    */
+  float monte_carlo_bias;  /* MONTE_CARLO_BIAS: diffuse ray origin = hit point + normal * bias             */
+  uint32_t seed;           /* Philox key word 0                                                            */
+  uint32_t frame_index;    /* Philox key word 1 (crtb200_render_frames: frame f uses frame_index + f)      */
+} crtb200_sampling;
+
+typedef struct crtb200_sampling_stats {
+  uint64_t rays_diffuse; /* DiffuseRay rays traced by the last render (not part of crtb200_stats)          */
+  uint32_t samples;      /* samples per pixel of the last render (1 with sampling off)                     */
+  uint32_t reserved;
+} crtb200_sampling_stats;
+
+/* replaces: RenderOptions::USE_GI / GI_SAMPLE_SIZE / RAYS_PER_PIXEL / MONTE_CARLO_BIAS (RayTracer.h:25-50) as passed to
+ * RayTracer::render.  Applies to every later render call of the context (like crtb200_set_concurrency); NULL or
+ * use_gi = 0 turns sampling off.  CRTB200_ERR_ARG when rays_per_pixel == 0 with GI on or gi_samples > 1024.  A frame
+ * whose ray tree (G^depth children per pixel) does not fit the queue budget fails with CRTB200_ERR_MEMORY. */
+int crtb200_set_sampling(crtb200_ctx *ctx, const crtb200_sampling *sampling);
+/* replaces: nothing in the reference (it counts no rays); the DiffuseRay count of RayTracer.cpp:331-354 */
+int crtb200_last_sampling_stats(crtb200_ctx *ctx, crtb200_sampling_stats *stats);
 
 /* replaces: the data RayTracer keeps in `scene`, `boundingBox`, `accelerationStructure` (RayTracer.h:64-67).
  * Copies + re-lays-out everything to device SoA during the call (host flattener H1). */

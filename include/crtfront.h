@@ -56,6 +56,12 @@ int crtfe_tracer_get_camera(crtfe_tracer *tracer, crtb200_camera *camera);
 /* RayTracer::render(pathToImage, RenderOptions{mode, max_depth, false}); rgb_out (optional) receives H*W*3 floats */
 int crtfe_tracer_render(crtfe_tracer *tracer, const char *path_to_image, uint32_t mode, uint32_t max_depth,
                         uint32_t literal_walk, float *rgb_out, crtb200_stats *stats);
+/* RayTracer::render(pathToImage, RenderOptions{mode, max_depth, use_gi, gi_samples, rays_per_pixel, ...,
+ * monte_carlo_bias}) with RenderOptions::SEED = seed: GI and jittered supersampling under the sampling contract of
+ * crtb200_set_sampling (frame_index 0) */
+int crtfe_tracer_render_sampled(crtfe_tracer *tracer, const char *path_to_image, uint32_t mode, uint32_t max_depth,
+                                uint32_t literal_walk, uint32_t use_gi, uint32_t gi_samples, uint32_t rays_per_pixel,
+                                float monte_carlo_bias, uint32_t seed, float *rgb_out, crtb200_stats *stats);
 
 #ifdef __cplusplus
 }
