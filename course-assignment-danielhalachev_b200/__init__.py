@@ -190,6 +190,12 @@ def core() -> C.CDLL:
         lib.crtb200_debug_powf5.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]
         lib.crtb200_set_sampling.argtypes = [C.c_void_p, C.POINTER(Sampling)]
         lib.crtb200_last_sampling_stats.argtypes = [C.c_void_p, C.POINTER(SamplingStats)]
+        lib.crtb200_accum_begin.argtypes = [C.c_void_p, C.POINTER(Camera), C.POINTER(Options), C.POINTER(Sampling)]
+        lib.crtb200_accum_step.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(Stats)]
+        lib.crtb200_accum_read.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_uint32)]
+        lib.crtb200_accum_save.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_uint32)]
+        lib.crtb200_accum_load.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32]
+        lib.crtb200_accum_end.argtypes = [C.c_void_p]
         _core = lib
     return _core
 
@@ -362,6 +368,7 @@ class Context:
             _check_core(core().crtb200_create(int(device), C.byref(self._h)))
         self.width = self.height = 0
         self._scene_keepalive = None
+        self._session = None  # the Progressive whose session the context holds
 
     def devices(self):
         n = C.c_int(0)
@@ -410,6 +417,32 @@ class Context:
                                           rgb8.ctypes.data if rgb8 is not None else None,
                                           hits.ctypes.data if hits is not None else None, C.byref(st)))
         return rgb, rgb8, hits, st.as_dict()
+
+    def progressive(self, camera: Camera, options: Options, sampling: Sampling) -> "Progressive":
+        """Begins a progressive GI session on the uploaded scene (crtb200_accum_begin); a session in progress ends."""
+        return Progressive(self, camera, options, sampling)
+
+    def resume(self, path: str, camera: Camera, options: Options, sampling: Sampling) -> "Progressive":
+        """Continues a session saved with Progressive.save on the scene this context holds.  camera, options and
+        sampling state what is to be continued: a file saved with another image size, camera, max_depth, biases,
+        rects or sampling (everything but rays_per_pixel) raises CrtError."""
+        with np.load(path, allow_pickle=False) as f:
+            data = {k: f[k] for k in f.files}
+        for k, v in _session_params(self.width, self.height, camera, options, sampling).items():
+            got = data.get(k)
+            if got is None or got.dtype != v.dtype or got.shape != v.shape or got.tobytes() != v.tobytes():
+                raise CrtError(f"{path}: the saved session's {k} differs from the session to continue")
+        h, w = self.height, self.width
+        arrays = {"sum": ((h, w, 3), np.float32), "sumsq": ((h, w, 3), np.float32), "hit0": ((h, w), HIT_DTYPE),
+                  "samples": ((), np.uint32)}
+        for k, (shape, dtype) in arrays.items():
+            if k not in data or data[k].shape != shape or data[k].dtype != dtype:
+                raise CrtError(f"{path}: {k} is missing or not {dtype} of shape {shape}")
+        p = Progressive(self, camera, options, sampling)
+        s, q, hit0 = (np.ascontiguousarray(data[k]) for k in ("sum", "sumsq", "hit0"))
+        _check_core(core().crtb200_accum_load(self._h, s.ctypes.data, q.ctypes.data, hit0.ctypes.data, int(data["samples"])))
+        p.samples = int(data["samples"])
+        return p
 
     def render_frames(self, cameras: Sequence[Camera], options: Options, want_rgb: bool = True, want_rgb8: bool = False):
         n = len(cameras)
@@ -485,6 +518,89 @@ class Context:
             self.close()
         except Exception:
             pass
+
+
+def _session_params(width: int, height: int, camera: Camera, options: Options, sampling: Sampling) -> dict:
+    """What a saved progressive session must agree on with the session that continues it (bit for bit)."""
+    rects = [(r.row, r.col, r.width, r.height) for r in options.rects[:options.n_rects]] if options.n_rects else []
+    return {
+        "size": np.array([height, width], np.uint32),
+        "camera": np.array(list(camera.position) + list(camera.rotation), np.float32),
+        "max_depth": np.array(options.max_depth, np.uint32),
+        "biases": np.array([options.shadow_bias, options.reflection_bias, options.refraction_bias], np.float32),
+        "rects": np.array(rects, np.uint32).reshape(-1, 4),
+        "sampling": np.array([sampling.use_gi, sampling.gi_samples, sampling.seed, sampling.frame_index], np.uint32),
+        "monte_carlo_bias": np.array(sampling.monte_carlo_bias, np.float32),
+    }
+
+
+class Progressive:
+    """A progressive GI session of a Context (crtb200_accum_*, DESIGN.md 3.10.1): samples accumulate in steps, and
+    after steps totalling n samples read() returns bit for bit the one-shot frame rendered with rays_per_pixel = n."""
+
+    def __init__(self, ctx: Context, camera: Camera, options: Options, sampling: Sampling):
+        self._ctx = ctx
+        self._params = _session_params(ctx.width, ctx.height, camera, options, sampling)
+        self.samples = 0
+        _check_core(core().crtb200_accum_begin(ctx._h, C.byref(camera), C.byref(options), C.byref(sampling)))
+        ctx._session = self
+
+    def _live(self):
+        if self._ctx._session is not self:
+            raise CrtError("this progressive session has ended (closed, or another one began on its context)")
+        return self._ctx._h
+
+    def step(self, n: int) -> dict:
+        """Renders n more samples per pixel; returns this step's stats (with rays_diffuse and samples)."""
+        if n < 0:
+            raise CrtError("n must not be negative")
+        st = Stats()
+        _check_core(core().crtb200_accum_step(self._live(), int(n), C.byref(st)))
+        self.samples += int(n)
+        d = st.as_dict()
+        d.update(self._ctx.sampling_stats())
+        return d
+
+    def read(self, want_rgb: bool = True, want_rgb8: bool = False, want_hits: bool = False):
+        """The image so far: (rgb f32 HxWx3 | None, rgb8 | None, sample 0's hits | None), laid out as Context.render's."""
+        h, w = self._ctx.height, self._ctx.width
+        rgb = np.zeros((h, w, 3), np.float32) if want_rgb else None
+        rgb8 = np.zeros((h, w, 3), np.uint8) if want_rgb8 else None
+        hits = np.zeros((h, w), HIT_DTYPE) if want_hits else None
+        _check_core(core().crtb200_accum_read(self._live(), rgb.ctypes.data if rgb is not None else None,
+                                              rgb8.ctypes.data if rgb8 is not None else None,
+                                              hits.ctypes.data if hits is not None else None, None))
+        return rgb, rgb8, hits
+
+    def arrays(self) -> dict:
+        """The accumulator: 'sum' and 'sumsq' (HxWx3 f32, 0 outside the rects), 'hit0' (sample 0's hits), 'samples'."""
+        h, w = self._ctx.height, self._ctx.width
+        s = np.zeros((h, w, 3), np.float32)
+        q = np.zeros((h, w, 3), np.float32)
+        hit0 = np.zeros((h, w), HIT_DTYPE)
+        n = C.c_uint32(0)
+        _check_core(core().crtb200_accum_save(self._live(), s.ctypes.data, q.ctypes.data, hit0.ctypes.data, C.byref(n)))
+        return {"sum": s, "sumsq": q, "hit0": hit0, "samples": np.uint32(n.value)}
+
+    def std_error(self) -> np.ndarray:
+        """Per-pixel, per-channel standard error of the mean, in float64: sqrt(max(0, (Q - S^2 / n) / (n - 1)) / n);
+        NaN below 2 samples.  An estimate of the noise left, not part of the bit-exact contract."""
+        a = self.arrays()
+        n = int(a["samples"])
+        if n < 2:
+            return np.full(a["sum"].shape, np.nan)
+        s, q = a["sum"].astype(np.float64), a["sumsq"].astype(np.float64)
+        return np.sqrt(np.maximum(0.0, (q - s * s / n) / (n - 1)) / n)
+
+    def save(self, path: str) -> None:
+        """Writes the accumulator and the session's parameters to an .npz file (Context.resume reads it)."""
+        np.savez(path, **self.arrays(), **self._params)
+
+    def close(self) -> None:
+        """Ends the session and frees its device memory (crtb200_accum_end)."""
+        if self._ctx._session is self:
+            _check_core(core().crtb200_accum_end(self._ctx._h))
+            self._ctx._session = None
 
 
 class RayTracer:

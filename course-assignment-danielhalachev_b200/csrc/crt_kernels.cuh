@@ -1536,6 +1536,111 @@ __global__ void __launch_bounds__(256) k_store(const DScene sc, const Frame fr, 
   }
 }
 
+// ------------------------------------------------------------------------------------------------------------
+// Progressive sessions (crtb200_accum_*, DESIGN.md 3.10.1).  The session's accumulator holds, per shard item (item_begin
+// + i, so that chunks never collide), S = ((0 + c_0) + c_1) + ..., Q = ((0 + c_0 c_0) + c_1 c_1) + ... and sample 0's
+// primary hit {global triangle, bits(t)}.  S and Q start at +0, so S is k_sample_acc's running sum bit for bit.
+// ------------------------------------------------------------------------------------------------------------
+// One sample pass of a session step, in place of k_sample_acc.  No k_store follows a step, so this counts the shadow
+// rays of every pass.
+__global__ void __launch_bounds__(256) k_accum_step(const DScene sc, const Frame fr, const Levels lv, float4 *__restrict__ sum,
+                                                   float4 *__restrict__ sumsq, uint2 *__restrict__ hit0) {
+  if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&lv.stats[1], (unsigned long long)lv.counts[CRT_MAX_LEVELS] * sc.n_lights);
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x) {
+    const uint32_t node = lv.offset[0] + i, k = fr.item_begin + i;
+    const float4 c = lv.color[node], s = sum[k], q = sumsq[k];
+    const V3 a = vadd(mk(s.x, s.y, s.z), mk(c.x, c.y, c.z));
+    const V3 b = vadd(mk(q.x, q.y, q.z), mk(fmul(c.x, c.x), fmul(c.y, c.y), fmul(c.z, c.z)));
+    sum[k] = make_float4(a.x, a.y, a.z, 0.f);
+    sumsq[k] = make_float4(b.x, b.y, b.z, 0.f);
+    if (fr.sample == 0) hit0[k] = make_uint2(lv.hit_tri[node], __float_as_uint(lv.hit_t[node]));
+  }
+}
+
+// Read: S / float(n) (k_sample_acc's division) and the kept hit into the level-0 slots, for k_store
+__global__ void __launch_bounds__(256) k_accum_read(const Frame fr, const Levels lv, const float4 *__restrict__ sum,
+                                                   const uint2 *__restrict__ hit0, uint32_t n_samples) {
+  const float n = (float)n_samples;
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x) {
+    const uint32_t node = lv.offset[0] + i, k = fr.item_begin + i;
+    const float4 s = sum[k];
+    const uint2 h = hit0[k];
+    lv.color[node] = make_float4(fdiv(s.x, n), fdiv(s.y, n), fdiv(s.z, n), 0.f);
+    lv.hit_tri[node] = h.x;
+    lv.hit_t[node] = __uint_as_float(h.y);
+  }
+}
+
+// Save: the accumulator of this chunk's covered pixels into frame-layout arrays (H*W*3 floats; public hit numbering,
+// mesh = triangle = -1 for a miss, t bits kept either way).  Any output may be null.
+__global__ void __launch_bounds__(256) k_accum_save(const DScene sc, const Frame fr, const float4 *__restrict__ sum,
+                                                   const float4 *__restrict__ sumsq, const uint2 *__restrict__ hit0,
+                                                   float *__restrict__ sum_out, float *__restrict__ sumsq_out,
+                                                   HitRec *__restrict__ hit_out) {
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x) {
+    uint32_t row, col;
+    if (!item_pixel(fr, sc, fr.item_begin + i, row, col)) continue;
+    const uint32_t k = fr.item_begin + i;
+    const size_t pix = (size_t)row * sc.width + col;
+    if (sum_out) {
+      const float4 s = sum[k];
+      sum_out[3 * pix + 0] = s.x;
+      sum_out[3 * pix + 1] = s.y;
+      sum_out[3 * pix + 2] = s.z;
+    }
+    if (sumsq_out) {
+      const float4 q = sumsq[k];
+      sumsq_out[3 * pix + 0] = q.x;
+      sumsq_out[3 * pix + 1] = q.y;
+      sumsq_out[3 * pix + 2] = q.z;
+    }
+    if (hit_out) {
+      const uint2 h = hit0[k];
+      HitRec r;
+      r.mesh = r.tri = -1;
+      if (h.x != CRT_INVALID) {
+        const uint32_t m = sc.tri_shade[h.x].w;
+        r.mesh = (int)m;
+        r.tri = (int)(h.x - sc.meshes[m].first_triangle);
+      }
+      r.t = __uint_as_float(h.y);
+      hit_out[pix] = r;
+    }
+  }
+}
+
+// Load: the reverse of k_accum_save.  The hit records come from a file: one that names no triangle of the uploaded
+// scene sets *bad and is not used.
+__global__ void __launch_bounds__(256) k_accum_load(const DScene sc, const Frame fr, const float *__restrict__ sum_in,
+                                                   const float *__restrict__ sumsq_in, const HitRec *__restrict__ hit_in,
+                                                   uint32_t n_triangles, float4 *__restrict__ sum, float4 *__restrict__ sumsq,
+                                                   uint2 *__restrict__ hit0, uint32_t *__restrict__ bad) {
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x) {
+    uint32_t row, col;
+    if (!item_pixel(fr, sc, fr.item_begin + i, row, col)) continue;
+    const uint32_t k = fr.item_begin + i;
+    const size_t pix = (size_t)row * sc.width + col;
+    sum[k] = make_float4(sum_in[3 * pix + 0], sum_in[3 * pix + 1], sum_in[3 * pix + 2], 0.f);
+    sumsq[k] = make_float4(sumsq_in[3 * pix + 0], sumsq_in[3 * pix + 1], sumsq_in[3 * pix + 2], 0.f);
+    const HitRec r = hit_in[pix];
+    uint32_t tri = CRT_INVALID;
+    if (r.mesh >= 0) {
+      const bool ok = (uint32_t)r.mesh < sc.n_meshes && r.tri >= 0 &&
+                      (unsigned long long)sc.meshes[r.mesh].first_triangle + (uint32_t)r.tri < n_triangles &&
+                      sc.tri_shade[sc.meshes[r.mesh].first_triangle + (uint32_t)r.tri].w == (uint32_t)r.mesh;
+      if (!ok) {
+        *bad = 1u;
+        continue;
+      }
+      tri = sc.meshes[r.mesh].first_triangle + (uint32_t)r.tri;
+    } else if (r.mesh != -1 || r.tri != -1) {
+      *bad = 1u;
+      continue;
+    }
+    hit0[k] = make_uint2(tri, __float_as_uint(r.t));
+  }
+}
+
 // Scatter gathered shard slabs (shard-major, item order) into a full frame: the rank-0 side of the NCCL gather.
 // A warp moves one 8x4 tile: 384 contiguous slab bytes in, four 96-byte frame rows out (16-byte accesses both ways when
 // the tile is whole and everything is aligned, like k_store).

@@ -239,6 +239,18 @@ struct crtb200_ctx {
   uint64_t last_diffuse = 0;  // diffuse rays of the last render (stats[41])
   uint32_t last_samples = 1;
   uint32_t cap_branch = 0;    // worst-case children per ray-tree node the queues were planned for
+  uint32_t n_triangles = 0;   // of the uploaded scene (crtb200_accum_load checks the hit records it is given)
+
+  // progressive session (crtb200_accum_*, DESIGN.md 3.10.1): the snapshots live on the primary, and every GPU of the
+  // context keeps the accumulator of its own tile shard, indexed by shard item
+  bool acc_active = false;
+  crtb200_camera acc_cam{};
+  crtb200_options acc_opt{};
+  std::vector<crtb200_rect> acc_rects;
+  crtb200_sampling acc_smp{};
+  uint32_t acc_done = 0;           // samples in the accumulator
+  DevBuf<float4> acc_sum, acc_sumsq;  // S and Q
+  DevBuf<uint2> acc_hit;              // sample 0's primary hit {global triangle, bits(t)}
 
   // multi-GPU (crtb200_create_multi): this context is the primary (device_ids[0]).  A frame's 8x4-pixel tiles are dealt
   // round-robin over primary + peers (scene replicated); every GPU's k_store writes its pixels STRAIGHT into the
@@ -389,6 +401,7 @@ int crtb200_destroy(crtb200_ctx *c) {
   c->tri_shade.release(); c->vtx_uv.release(); c->meshes.release(); c->materials.release(); c->textures.release();
   c->texels.release(); c->lights.release(); c->frame.release(); c->frame8.release(); c->hits.release();
   c->mask.release(); c->frame_b.release(); c->frame8_b.release();
+  c->acc_sum.release(); c->acc_sumsq.release(); c->acc_hit.release();
   if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
   for (int k = 0; k < 2; k++) {
     if (c->rendered[k]) cudaEventDestroy(c->rendered[k]);
@@ -617,6 +630,21 @@ static float mesh_cull_margin(const crtb200_scene *s, const crtb200_mesh &me, bo
 
 static int upload_one(crtb200_ctx *c, const crtb200_scene *s);
 
+// ends the progressive session of a context and frees its accumulators on every GPU
+static void accum_release(crtb200_ctx *c) {
+  c->acc_active = false;
+  c->acc_done = 0;
+  c->acc_rects.clear();
+  for (size_t i = 0; i <= c->peers.size(); i++) {
+    crtb200_ctx *x = i ? c->peers[i - 1] : c;
+    cudaSetDevice(x->device);
+    x->acc_sum.release();
+    x->acc_sumsq.release();
+    x->acc_hit.release();
+  }
+  cudaSetDevice(c->device);
+}
+
 // runs fn(peer index, peer) on every peer's helper thread and fn0 on the calling thread; first error wins
 template <typename F0, typename F>
 static int on_all_devices(crtb200_ctx *c, F0 fn0, F fn) {
@@ -640,6 +668,7 @@ extern "C" {
 int crtb200_upload_scene(crtb200_ctx *c, const crtb200_scene *s) {
   if (!c || !s) return fail(CRTB200_ERR_ARG, "null argument");
   ErrScope scope(c);
+  if (c->acc_active) accum_release(c);  // a new scene ends the progressive session
   if (c->peers.empty()) return upload_one(c, s);
   // scene replicated on every GPU (SURVEY 8(e)); the host relayout runs once per GPU, in parallel
   return on_all_devices(c, [&] { return upload_one(c, s); }, [&](size_t, crtb200_ctx *p) { return upload_one(p, s); });
@@ -806,6 +835,7 @@ static int upload_one(crtb200_ctx *c, const crtb200_scene *s) {
   CUDA_TRY(c->texels.upload(texels));
   CUDA_TRY(c->lights.upload(lights));
   c->scene_bytes = nodes.size() * 16 + refs.size() * 4 + geom.size() * 16 + shade.size() * 16 + vn.size() * 16;
+  c->n_triangles = s->n_triangles;
 
   DScene &d = c->sc;
   d.nodes = c->nodes_p;
@@ -1105,10 +1135,23 @@ struct HostOut {
   crtb200_hit *hits = nullptr;
 };
 
+// A pass of a progressive session (DESIGN.md 3.10.1) through the chunk loop of enqueue_frame, on the accumulator of the
+// context it runs on.  STEP renders global samples [s0, s0 + n) into it; READ stores S / float(s0) and the kept hit
+// through k_store; SAVE / LOAD move it to / from frame-layout arrays in the primary's memory (peer-mapped on the other
+// GPUs of a multi-GPU context, like k_store's frame).  No pass but STEP runs a sample.
+struct AccumPass {
+  enum Mode { STEP, READ, SAVE, LOAD } mode;
+  uint32_t s0, n;
+  float *px_sum, *px_sumsq;
+  HitRec *px_hit;
+  uint32_t *bad;  // LOAD: set when a hit record names no triangle of the scene
+};
+
 // Enqueue one frame on `st`.  d_rgb / d_rgb8 / d_hits / d_slab are device pointers (any may be null).
 static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_options *o, float *d_rgb,
                          uint8_t *d_rgb8, HitRec *d_hits, float *d_slab, cudaStream_t st, bool timed,
-                         const HostOut *host = nullptr, bool *host_done = nullptr, bool batch_continuation = false) {
+                         const HostOut *host = nullptr, bool *host_done = nullptr, bool batch_continuation = false,
+                         const AccumPass *acc = nullptr) {
   if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
   if (o->max_depth > 31) return fail(CRTB200_ERR_ARG, "max_depth > 31 is not supported");
   if (o->n_rects && !o->rects) return fail(CRTB200_ERR_ARG, "n_rects > 0 but rects is null");
@@ -1152,7 +1195,8 @@ static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb20
   if (rc) return rc;
   const bool secondary = c->has_reflective || c->has_refractive || gi;
   const uint32_t levels = secondary ? o->max_depth + 1 : 1;
-  c->last_samples = fr.spp;
+  c->last_samples = acc ? acc->n : fr.spp;
+  const uint32_t s_begin = acc ? acc->s0 : 0u, s_end = acc ? acc->s0 + acc->n : fr.spp;
   // Band copies need chunks that own whole rows of tiles: with a small queue budget or a deep refractive scene a chunk
   // is smaller than a tile row, two chunks on different streams would then share a 4-row band and a band copy could
   // pick up the other chunk's stale pixels.  Then the caller copies the whole frame after the join instead.
@@ -1192,11 +1236,11 @@ static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb20
     cudaStream_t qs = q.stream;
     fr.item_begin = begin;
     fr.n_items0 = std::min(c->cap_items, shard_items - begin);
-    if (gi) {
+    if (gi && !acc) {
       CUDA_TRY(q.acc.ensure(c->cap_items));
       CUDA_TRY(q.hit0.ensure(c->cap_items));
     }
-    for (uint32_t s = 0; s < fr.spp; s++) {
+    for (uint32_t s = s_begin; s < s_end; s++) {
       fr.sample = s;
       CUDA_TRY(cudaMemsetAsync(q.ctl.p, 0, q.ctl.n * sizeof(uint32_t), qs));
       q.lv.tail_iters = handoff ? (uint32_t)(c->tail_iters + 1) : 0u;
@@ -1273,13 +1317,31 @@ static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb20
           k_resolve<false><<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, l);
         launches++;
       }
-      if (gi) {
+      if (acc) {
+        k_accum_step<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p);
+        launches++;
+      } else if (gi) {
         k_sample_acc<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, q.acc.p, q.hit0.p);
         launches++;
       }
     }
-    k_store<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, d_rgb, d_rgb8, d_hits, d_slab);
-    launches++;
+    if (acc && acc->mode == AccumPass::READ) {
+      CUDA_TRY(cudaMemsetAsync(q.ctl.p, 0, q.ctl.n * sizeof(uint32_t), qs));  // k_store then counts no shadow rays
+      k_accum_read<<<grid_simple, 256, 0, qs>>>(fr, q.lv, c->acc_sum.p, c->acc_hit.p, acc->s0);
+      launches++;
+    } else if (acc && acc->mode == AccumPass::SAVE) {
+      k_accum_save<<<grid_simple, 256, 0, qs>>>(c->sc, fr, c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p, acc->px_sum,
+                                                acc->px_sumsq, acc->px_hit);
+      launches++;
+    } else if (acc && acc->mode == AccumPass::LOAD) {
+      k_accum_load<<<grid_simple, 256, 0, qs>>>(c->sc, fr, acc->px_sum, acc->px_sumsq, acc->px_hit, c->n_triangles,
+                                                c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p, acc->bad);
+      launches++;
+    }
+    if (!acc || acc->mode == AccumPass::READ) {
+      k_store<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, d_rgb, d_rgb8, d_hits, d_slab);
+      launches++;
+    }
     if (band_copies) {
       const uint32_t row0 = (begin / row_items) * 4u;
       const uint32_t row1 = std::min<uint32_t>(H, ((begin + fr.n_items0 + row_items - 1) / row_items) * 4u);
@@ -1325,9 +1387,9 @@ static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb20
 // (earlier consumers of the frame on the primary's stream are done) and `st` continues after every peer has stored.
 static int enqueue_any(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_options *o, float *d_rgb, uint8_t *d_rgb8,
                        HitRec *d_hits, float *d_slab, cudaStream_t st, bool timed, const HostOut *host = nullptr,
-                       bool *host_done = nullptr, bool batch_continuation = false) {
+                       bool *host_done = nullptr, bool batch_continuation = false, const AccumPass *acc = nullptr) {
   if (c->peers.empty() || o->shard_count > 1)
-    return enqueue_frame(c, cam, o, d_rgb, d_rgb8, d_hits, d_slab, st, timed, host, host_done, batch_continuation);
+    return enqueue_frame(c, cam, o, d_rgb, d_rgb8, d_hits, d_slab, st, timed, host, host_done, batch_continuation, acc);
   if (host_done) *host_done = false;  // the caller copies the assembled frame after the join
   const uint32_t n = 1u + (uint32_t)c->peers.size();
   CUDA_TRY(cudaSetDevice(c->device));
@@ -1336,14 +1398,14 @@ static int enqueue_any(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_
   o0.shard_index = 0;
   o0.shard_count = n;
   int rc = on_all_devices(
-      c, [&] { return enqueue_frame(c, cam, &o0, d_rgb, d_rgb8, d_hits, nullptr, st, timed, nullptr, nullptr, batch_continuation); },
+      c, [&] { return enqueue_frame(c, cam, &o0, d_rgb, d_rgb8, d_hits, nullptr, st, timed, nullptr, nullptr, batch_continuation, acc); },
       [&](size_t i, crtb200_ctx *p) {
         crtb200_options oi = *o;
         oi.shard_index = (uint32_t)i + 1u;
         oi.shard_count = n;
         CUDA_TRY(cudaSetDevice(p->device));
         CUDA_TRY(cudaStreamWaitEvent(p->stream, c->multi_fork, 0));
-        int r = enqueue_frame(p, cam, &oi, d_rgb, d_rgb8, d_hits, nullptr, p->stream, true, nullptr, nullptr, batch_continuation);
+        int r = enqueue_frame(p, cam, &oi, d_rgb, d_rgb8, d_hits, nullptr, p->stream, true, nullptr, nullptr, batch_continuation, acc);
         if (r) return r;
         p->last_pending = true;
         CUDA_TRY(cudaEventRecord(p->multi_done, p->stream));
@@ -1635,6 +1697,200 @@ int crtb200_render_device(crtb200_ctx *c, const crtb200_camera *cam, const crtb2
     return enqueue_frame(c, cam, o, nullptr, nullptr, nullptr, d_rgb_out, (cudaStream_t)stream, true);
   }
   return enqueue_any(c, cam, o, d_rgb_out, d_rgb8_out, nullptr, nullptr, (cudaStream_t)stream, true);
+}
+
+// ---- progressive sessions (DESIGN.md 3.10.1) ---------------------------------------------------------------------
+// One session pass on every GPU of the context, with the session's snapshots.  The session's sampling stands in for the
+// context's for the call, because queue planning and the Philox key both read ctx->sampling; frame_offset is 0 outside
+// crtb200_render_frames, so the key is the session's frame_index.
+static int session_pass(crtb200_ctx *c, const AccumPass &a, float *d_rgb, uint8_t *d_rgb8, HitRec *d_hits, bool timed) {
+  std::vector<crtb200_sampling> saved;
+  for (size_t i = 0; i <= c->peers.size(); i++) {
+    crtb200_ctx *x = i ? c->peers[i - 1] : c;
+    saved.push_back(x->sampling);
+    x->sampling = c->acc_smp;
+  }
+  const int rc = enqueue_any(c, &c->acc_cam, &c->acc_opt, d_rgb, d_rgb8, d_hits, nullptr, c->stream, timed, nullptr, nullptr, false, &a);
+  for (size_t i = 0; i <= c->peers.size(); i++) (i ? c->peers[i - 1] : c)->sampling = saved[i];
+  return rc;
+}
+
+// device staging of a save / load: frame-layout S, Q and hit records on the primary
+struct AccumStaging {
+  DevBuf<float> sum, sumsq;
+  DevBuf<HitRec> hit;
+  DevBuf<uint32_t> bad;
+  ~AccumStaging() {
+    sum.release();
+    sumsq.release();
+    hit.release();
+    bad.release();
+  }
+};
+
+int crtb200_accum_begin(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_options *o, const crtb200_sampling *s) {
+  ErrScope scope(c);
+  if (!c || !cam || !o || !s) return fail(CRTB200_ERR_ARG, "null argument");
+  CUDA_TRY(cudaSetDevice(c->device));
+  if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
+  if (!s->use_gi) return fail(CRTB200_ERR_ARG, "a progressive session needs sampling.use_gi = 1");
+  if (s->gi_samples > 1024) return fail(CRTB200_ERR_ARG, "gi_samples must be at most 1024");
+  if (o->shard_count > 1 || o->shard_index != 0)
+    return fail(CRTB200_ERR_ARG, "progressive sessions are not tile-sharded (several GPUs: crtb200_create_multi)");
+  if (o->max_depth > 31 || (o->n_rects && !o->rects) || o->traversal > 1 || o->count_work > 2)
+    return fail(CRTB200_ERR_ARG, "bad options (max_depth > 31, null rects, or unknown traversal / count_work mode)");
+  accum_release(c);
+  c->acc_cam = *cam;
+  c->acc_opt = *o;
+  c->acc_rects.assign(o->rects, o->rects + o->n_rects);
+  c->acc_opt.rects = o->n_rects ? c->acc_rects.data() : nullptr;
+  c->acc_smp = *s;
+  c->acc_smp.use_gi = 1;
+  c->acc_smp.rays_per_pixel = 1;  // unused: a step says how many samples it renders
+  const uint32_t n = 1u + (uint32_t)c->peers.size();
+  const uint32_t tiles = ((c->sc.width + 7) / 8) * ((c->sc.height + 3) / 4);
+  for (uint32_t i = 0; i < n; i++) {
+    crtb200_ctx *x = i ? c->peers[i - 1] : c;
+    const size_t items = std::max<size_t>(1, (size_t)(tiles > i ? (tiles - i + n - 1) / n : 0) * 32u);  // shard i of n
+    cudaError_t e = cudaSetDevice(x->device);
+    if (e == cudaSuccess) e = x->acc_sum.ensure(items);
+    if (e == cudaSuccess) e = x->acc_sumsq.ensure(items);
+    if (e == cudaSuccess) e = x->acc_hit.ensure(items);
+    if (e == cudaSuccess) e = cudaMemsetAsync(x->acc_sum.p, 0, items * sizeof(float4), x->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(x->acc_sumsq.p, 0, items * sizeof(float4), x->stream);
+    // no hit until sample 0 has run: a save at 0 samples must not look up a triangle
+    if (e == cudaSuccess) e = cudaMemsetAsync(x->acc_hit.p, 0xFF, items * sizeof(uint2), x->stream);
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      accum_release(c);
+      return fail(e == cudaErrorMemoryAllocation ? CRTB200_ERR_MEMORY : CRTB200_ERR_CUDA,
+                  std::string("progressive accumulator (40 bytes per pixel) on device ") + std::to_string(x->device) + ": " +
+                      cudaGetErrorString(e));
+    }
+  }
+  CUDA_TRY(cudaSetDevice(c->device));
+  c->acc_active = true;
+  return CRTB200_OK;
+}
+
+int crtb200_accum_step(crtb200_ctx *c, uint32_t n_samples, crtb200_stats *stats) {
+  ErrScope scope(c);
+  if (!c) return fail(CRTB200_ERR_ARG, "ctx is null");
+  CUDA_TRY(cudaSetDevice(c->device));
+  if (!c->acc_active) return fail(CRTB200_ERR_STATE, "no progressive session (crtb200_accum_begin)");
+  if (n_samples == 0 || (uint64_t)c->acc_done + n_samples > 0xFFFFFFFFull) return fail(CRTB200_ERR_ARG, "n_samples must be at least 1");
+  const auto t0 = std::chrono::steady_clock::now();
+  c->last = crtb200_stats{};
+  const AccumPass a{AccumPass::STEP, c->acc_done, n_samples, nullptr, nullptr, nullptr, nullptr};
+  int rc = session_pass(c, a, nullptr, nullptr, nullptr, true);
+  if (rc) return rc;
+  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  rc = collect_stats(c, true);
+  if (rc) return rc;
+  c->acc_done += n_samples;
+  c->last.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+  if (stats) *stats = c->last;
+  return CRTB200_OK;
+}
+
+int crtb200_accum_read(crtb200_ctx *c, float *rgb_out, uint8_t *rgb8_out, crtb200_hit *hits_out, uint32_t *samples_done) {
+  ErrScope scope(c);
+  if (!c) return fail(CRTB200_ERR_ARG, "ctx is null");
+  CUDA_TRY(cudaSetDevice(c->device));
+  if (!c->acc_active) return fail(CRTB200_ERR_STATE, "no progressive session (crtb200_accum_begin)");
+  if (c->acc_done == 0) return fail(CRTB200_ERR_STATE, "the progressive session has no samples yet");
+  const size_t px = (size_t)c->sc.width * c->sc.height;
+  if (hits_out) CUDA_TRY(c->hits.ensure(px));
+  if (hits_out) CUDA_TRY(cudaMemsetAsync(c->hits.p, 0xFF, px * sizeof(HitRec), c->stream));
+  // a read is no render: the last render's statistics stay what they were
+  const crtb200_stats keep = c->last;
+  const uint32_t keep_samples = c->last_samples;
+  const AccumPass a{AccumPass::READ, c->acc_done, 0, nullptr, nullptr, nullptr, nullptr};
+  const int rc = session_pass(c, a, c->frame.p, rgb8_out ? c->frame8.p : nullptr, hits_out ? c->hits.p : nullptr, false);
+  c->last = keep;
+  c->last_samples = keep_samples;
+  if (rc) return rc;
+  if (rgb_out) CUDA_TRY(cudaMemcpyAsync(rgb_out, c->frame.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  if (rgb8_out) CUDA_TRY(cudaMemcpyAsync(rgb8_out, c->frame8.p, px * 3, cudaMemcpyDeviceToHost, c->stream));
+  if (hits_out) CUDA_TRY(cudaMemcpyAsync(hits_out, c->hits.p, px * sizeof(HitRec), cudaMemcpyDeviceToHost, c->stream));
+  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  if (samples_done) *samples_done = c->acc_done;
+  return CRTB200_OK;
+}
+
+int crtb200_accum_save(crtb200_ctx *c, float *sum_out, float *sumsq_out, crtb200_hit *hit0_out, uint32_t *samples_done) {
+  ErrScope scope(c);
+  if (!c) return fail(CRTB200_ERR_ARG, "ctx is null");
+  CUDA_TRY(cudaSetDevice(c->device));
+  if (!c->acc_active) return fail(CRTB200_ERR_STATE, "no progressive session (crtb200_accum_begin)");
+  const size_t px = (size_t)c->sc.width * c->sc.height;
+  AccumStaging g;
+  if (sum_out) {
+    CUDA_TRY(g.sum.ensure(px * 3));
+    CUDA_TRY(cudaMemsetAsync(g.sum.p, 0, px * 3 * sizeof(float), c->stream));
+  }
+  if (sumsq_out) {
+    CUDA_TRY(g.sumsq.ensure(px * 3));
+    CUDA_TRY(cudaMemsetAsync(g.sumsq.p, 0, px * 3 * sizeof(float), c->stream));
+  }
+  if (hit0_out) {
+    CUDA_TRY(g.hit.ensure(px));
+    CUDA_TRY(cudaMemsetAsync(g.hit.p, 0xFF, px * sizeof(HitRec), c->stream));
+  }
+  const crtb200_stats keep = c->last;
+  const uint32_t keep_samples = c->last_samples;
+  const AccumPass a{AccumPass::SAVE, c->acc_done, 0, g.sum.p, g.sumsq.p, g.hit.p, nullptr};
+  const int rc = session_pass(c, a, nullptr, nullptr, nullptr, false);
+  c->last = keep;
+  c->last_samples = keep_samples;
+  if (rc) return rc;
+  if (sum_out) CUDA_TRY(cudaMemcpyAsync(sum_out, g.sum.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  if (sumsq_out) CUDA_TRY(cudaMemcpyAsync(sumsq_out, g.sumsq.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  if (hit0_out) CUDA_TRY(cudaMemcpyAsync(hit0_out, g.hit.p, px * sizeof(HitRec), cudaMemcpyDeviceToHost, c->stream));
+  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  if (samples_done) *samples_done = c->acc_done;
+  return CRTB200_OK;
+}
+
+int crtb200_accum_load(crtb200_ctx *c, const float *sum, const float *sumsq, const crtb200_hit *hit0, uint32_t samples_done) {
+  ErrScope scope(c);
+  if (!c || !sum || !sumsq || !hit0) return fail(CRTB200_ERR_ARG, "null argument");
+  CUDA_TRY(cudaSetDevice(c->device));
+  if (!c->acc_active) return fail(CRTB200_ERR_STATE, "no progressive session (crtb200_accum_begin)");
+  const size_t px = (size_t)c->sc.width * c->sc.height;
+  AccumStaging g;
+  CUDA_TRY(g.sum.ensure(px * 3));
+  CUDA_TRY(g.sumsq.ensure(px * 3));
+  CUDA_TRY(g.hit.ensure(px));
+  CUDA_TRY(g.bad.ensure(1));
+  CUDA_TRY(cudaMemcpyAsync(g.sum.p, sum, px * 3 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+  CUDA_TRY(cudaMemcpyAsync(g.sumsq.p, sumsq, px * 3 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+  CUDA_TRY(cudaMemcpyAsync(g.hit.p, hit0, px * sizeof(HitRec), cudaMemcpyHostToDevice, c->stream));
+  CUDA_TRY(cudaMemsetAsync(g.bad.p, 0, sizeof(uint32_t), c->stream));
+  const crtb200_stats keep = c->last;
+  const uint32_t keep_samples = c->last_samples;
+  const AccumPass a{AccumPass::LOAD, 0, 0, g.sum.p, g.sumsq.p, g.hit.p, g.bad.p};
+  const int rc = session_pass(c, a, nullptr, nullptr, nullptr, false);
+  c->last = keep;
+  c->last_samples = keep_samples;
+  if (rc) return rc;
+  uint32_t bad = 0;
+  CUDA_TRY(cudaMemcpyAsync(&bad, g.bad.p, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  if (bad) {
+    accum_release(c);
+    return fail(CRTB200_ERR_ARG, "hit records name triangles the uploaded scene does not have; the session has ended");
+  }
+  c->acc_done = samples_done;
+  return CRTB200_OK;
+}
+
+int crtb200_accum_end(crtb200_ctx *c) {
+  ErrScope scope(c);
+  if (!c) return fail(CRTB200_ERR_ARG, "ctx is null");
+  CUDA_TRY(cudaSetDevice(c->device));
+  accum_release(c);
+  return CRTB200_OK;
 }
 
 int crtb200_last_stats(crtb200_ctx *c, crtb200_stats *stats) {

@@ -254,6 +254,43 @@ int crtb200_set_sampling(crtb200_ctx *ctx, const crtb200_sampling *sampling);
 /* replaces: nothing in the reference (it counts no rays); the DiffuseRay count of RayTracer.cpp:331-354 */
 int crtb200_last_sampling_stats(crtb200_ctx *ctx, crtb200_sampling_stats *stats);
 
+/* Progressive sessions (DESIGN.md 3.10.1): a GI frame rendered in steps of samples, readable after any step, saved and
+ * resumed.  None of these has a counterpart in the reference: RayTracer::render runs all RAYS_PER_PIXEL samples of a
+ * pixel in one loop and keeps no running sum (RayTracer.cpp:90-104).  One session per context; it holds a persistent
+ * per-pixel accumulator of 40 bytes per pixel on each GPU (that GPU's tile shard).  After steps totalling n samples,
+ * crtb200_accum_read returns bit for bit what crtb200_render returns with the same camera and options and
+ * rays_per_pixel = n, and the steps' ray counts (and, with count_work = 1, test counts) add up to that frame's.
+ * Ordinary renders and crtb200_set_sampling between steps do not affect the session; crtb200_upload_scene and
+ * crtb200_destroy end it.  Every call but begin fails with CRTB200_ERR_STATE without a session. */
+
+/* replaces: the per-pixel sample loop's set-up, RayTracer.cpp:90-104 (no counterpart: see above).  Snapshots camera,
+ * options (the rects array is copied) and sampling (rays_per_pixel is ignored) and starts at 0 samples; a session in
+ * progress ends.  CRTB200_ERR_ARG when use_gi = 0 or options->shard_count > 1 (several GPUs: crtb200_create_multi);
+ * CRTB200_ERR_MEMORY when the accumulator does not fit on a device. */
+int crtb200_accum_begin(crtb200_ctx *ctx, const crtb200_camera *camera, const crtb200_options *options,
+                        const crtb200_sampling *sampling);
+/* replaces: n_samples more iterations of the sample loop of RayTracer.cpp:90-104 (no counterpart: see above).  Renders
+ * samples [done, done + n_samples) of every covered pixel exactly as a one-shot frame renders them, accumulating
+ * S = S + c and Q = Q + c * c per channel in sample order.  stats (optional) and crtb200_last_stats /
+ * crtb200_last_sampling_stats describe this step.  CRTB200_ERR_ARG when n_samples == 0. */
+int crtb200_accum_step(crtb200_ctx *ctx, uint32_t n_samples, crtb200_stats *stats);
+/* replaces: the division by RAYS_PER_PIXEL and the colorBuffer store after the loop, RayTracer.cpp:90-106 (no
+ * counterpart: see above).  S / float(samples) into rgb_out / rgb8_out and sample 0's primary hit into hits_out, each
+ * optional and laid out as in crtb200_render; pixels outside the session's rects keep the context's colour buffer, as
+ * crtb200_render leaves them.  CRTB200_ERR_STATE at 0 samples.  Adds nothing to the statistics. */
+int crtb200_accum_read(crtb200_ctx *ctx, float *rgb_out, uint8_t *rgb8_out, crtb200_hit *hits_out, uint32_t *samples_done);
+/* replaces: nothing in the reference (see above).  sum_out / sumsq_out: S and Q, H*W*3 float32 row-major, 0 outside
+ * the rects; hit0_out: H*W sample-0 hits (mesh = triangle = -1 for a miss and outside the rects; t bits as traced).
+ * Each optional. */
+int crtb200_accum_save(crtb200_ctx *ctx, float *sum_out, float *sumsq_out, crtb200_hit *hit0_out, uint32_t *samples_done);
+/* replaces: nothing in the reference (see above).  The reverse of crtb200_accum_save, on a session begun with the same
+ * camera, options and sampling: later steps continue as if the saved samples had been rendered here.  Pixels outside
+ * the rects are not read.  CRTB200_ERR_ARG, and the session ends, when a hit names no triangle of the scene. */
+int crtb200_accum_load(crtb200_ctx *ctx, const float *sum, const float *sumsq, const crtb200_hit *hit0,
+                       uint32_t samples_done);
+/* replaces: nothing in the reference (see above).  Ends the session and frees its accumulators; no-op without one. */
+int crtb200_accum_end(crtb200_ctx *ctx);
+
 /* replaces: the data RayTracer keeps in `scene`, `boundingBox`, `accelerationStructure` (RayTracer.h:64-67).
  * Copies + re-lays-out everything to device SoA during the call (host flattener H1). */
 int crtb200_upload_scene(crtb200_ctx *ctx, const crtb200_scene *scene);
