@@ -134,6 +134,20 @@ class Sampling(C.Structure):
         return Sampling(1 if use_gi else 0, gi_samples, rays_per_pixel, monte_carlo_bias, seed, frame_index)
 
 
+class Adaptive(C.Structure):
+    """crtb200_adaptive: the stop rule of an adaptive progressive session (DESIGN.md 3.10.2)."""
+    _fields_ = [("min_samples", C.c_uint32), ("max_samples", C.c_uint32), ("abs_error", C.c_float), ("rel_error", C.c_float)]
+
+    @staticmethod
+    def make(min_samples: int = 8, max_samples: int = 128, abs_error: float = 0.0, rel_error: float = 0.05) -> "Adaptive":
+        return Adaptive(min_samples, max_samples, abs_error, rel_error)
+
+
+class AccumProgress(C.Structure):
+    _fields_ = [("passes", C.c_uint32), ("reserved", C.c_uint32), ("covered_pixels", C.c_uint64),
+                ("active_pixels", C.c_uint64), ("pixel_samples", C.c_uint64)]
+
+
 class SamplingStats(C.Structure):
     _fields_ = [("rays_diffuse", C.c_uint64), ("samples", C.c_uint32), ("reserved", C.c_uint32)]
 
@@ -196,6 +210,11 @@ def core() -> C.CDLL:
         lib.crtb200_accum_save.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_uint32)]
         lib.crtb200_accum_load.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32]
         lib.crtb200_accum_end.argtypes = [C.c_void_p]
+        lib.crtb200_accum_begin_adaptive.argtypes = [C.c_void_p, C.POINTER(Camera), C.POINTER(Options), C.POINTER(Sampling),
+                                                     C.POINTER(Adaptive)]
+        lib.crtb200_accum_progress.argtypes = [C.c_void_p, C.POINTER(AccumProgress)]
+        lib.crtb200_accum_counts.argtypes = [C.c_void_p, C.c_void_p]
+        lib.crtb200_accum_load_counts.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32]
         _core = lib
     return _core
 
@@ -418,29 +437,45 @@ class Context:
                                           hits.ctypes.data if hits is not None else None, C.byref(st)))
         return rgb, rgb8, hits, st.as_dict()
 
-    def progressive(self, camera: Camera, options: Options, sampling: Sampling) -> "Progressive":
-        """Begins a progressive GI session on the uploaded scene (crtb200_accum_begin); a session in progress ends."""
-        return Progressive(self, camera, options, sampling)
+    def progressive(self, camera: Camera, options: Options, sampling: Sampling,
+                    adaptive: Optional[Adaptive] = None) -> "Progressive":
+        """Begins a progressive GI session on the uploaded scene (crtb200_accum_begin, or with `adaptive`
+        crtb200_accum_begin_adaptive); a session in progress ends."""
+        return Progressive(self, camera, options, sampling, adaptive)
 
-    def resume(self, path: str, camera: Camera, options: Options, sampling: Sampling) -> "Progressive":
-        """Continues a session saved with Progressive.save on the scene this context holds.  camera, options and
-        sampling state what is to be continued: a file saved with another image size, camera, max_depth, biases,
-        rects or sampling (everything but rays_per_pixel) raises CrtError."""
+    def resume(self, path: str, camera: Camera, options: Options, sampling: Sampling,
+               adaptive: Optional[Adaptive] = None) -> "Progressive":
+        """Continues a session saved with Progressive.save on the scene this context holds.  camera, options,
+        sampling and adaptive state what is to be continued: a file saved with another image size, camera, max_depth,
+        biases, rects, sampling (everything but rays_per_pixel) or stop rule, or an adaptive file for a plain session
+        and the reverse, raises CrtError."""
         with np.load(path, allow_pickle=False) as f:
             data = {k: f[k] for k in f.files}
         for k, v in _session_params(self.width, self.height, camera, options, sampling).items():
             got = data.get(k)
             if got is None or got.dtype != v.dtype or got.shape != v.shape or got.tobytes() != v.tobytes():
                 raise CrtError(f"{path}: the saved session's {k} differs from the session to continue")
+        if ("adaptive" in data) != (adaptive is not None) or ("counts" in data) != (adaptive is not None):
+            raise CrtError(f"{path}: the saved session is {'adaptive' if 'adaptive' in data else 'plain'}, the session "
+                           f"to continue is {'adaptive' if adaptive is not None else 'plain'}")
+        if adaptive is not None and data["adaptive"].tobytes() != _adaptive_param(adaptive).tobytes():
+            raise CrtError(f"{path}: the saved session's adaptive parameters differ from the session to continue")
         h, w = self.height, self.width
         arrays = {"sum": ((h, w, 3), np.float32), "sumsq": ((h, w, 3), np.float32), "hit0": ((h, w), HIT_DTYPE),
                   "samples": ((), np.uint32)}
+        if adaptive is not None:
+            arrays["counts"] = ((h, w), np.uint32)
         for k, (shape, dtype) in arrays.items():
             if k not in data or data[k].shape != shape or data[k].dtype != dtype:
                 raise CrtError(f"{path}: {k} is missing or not {dtype} of shape {shape}")
-        p = Progressive(self, camera, options, sampling)
+        p = Progressive(self, camera, options, sampling, adaptive)
         s, q, hit0 = (np.ascontiguousarray(data[k]) for k in ("sum", "sumsq", "hit0"))
-        _check_core(core().crtb200_accum_load(self._h, s.ctypes.data, q.ctypes.data, hit0.ctypes.data, int(data["samples"])))
+        if adaptive is None:
+            _check_core(core().crtb200_accum_load(self._h, s.ctypes.data, q.ctypes.data, hit0.ctypes.data, int(data["samples"])))
+        else:
+            counts = np.ascontiguousarray(data["counts"])
+            _check_core(core().crtb200_accum_load_counts(self._h, s.ctypes.data, q.ctypes.data, hit0.ctypes.data,
+                                                         counts.ctypes.data, int(data["samples"])))
         p.samples = int(data["samples"])
         return p
 
@@ -534,15 +569,31 @@ def _session_params(width: int, height: int, camera: Camera, options: Options, s
     }
 
 
+def _adaptive_param(adaptive: Adaptive) -> np.ndarray:
+    """The stop rule as saved with an adaptive session: min, max and the bits of abs_error, rel_error."""
+    return np.array([adaptive.min_samples, adaptive.max_samples, np.float32(adaptive.abs_error).view(np.uint32),
+                     np.float32(adaptive.rel_error).view(np.uint32)], np.uint32)
+
+
 class Progressive:
     """A progressive GI session of a Context (crtb200_accum_*, DESIGN.md 3.10.1): samples accumulate in steps, and
-    after steps totalling n samples read() returns bit for bit the one-shot frame rendered with rays_per_pixel = n."""
+    after steps totalling n samples read() returns bit for bit the one-shot frame rendered with rays_per_pixel = n.
+    An adaptive session (DESIGN.md 3.10.2) stops each pixel once its noise is below the Adaptive bound: pixel p of a
+    read is then the one-shot frame's pixel p with rays_per_pixel = counts()[p].  `samples` counts passes."""
 
-    def __init__(self, ctx: Context, camera: Camera, options: Options, sampling: Sampling):
+    def __init__(self, ctx: Context, camera: Camera, options: Options, sampling: Sampling,
+                 adaptive: Optional[Adaptive] = None):
         self._ctx = ctx
         self._params = _session_params(ctx.width, ctx.height, camera, options, sampling)
+        self.adaptive = adaptive
+        if adaptive is not None:
+            self._params["adaptive"] = _adaptive_param(adaptive)
         self.samples = 0
-        _check_core(core().crtb200_accum_begin(ctx._h, C.byref(camera), C.byref(options), C.byref(sampling)))
+        if adaptive is None:
+            _check_core(core().crtb200_accum_begin(ctx._h, C.byref(camera), C.byref(options), C.byref(sampling)))
+        else:
+            _check_core(core().crtb200_accum_begin_adaptive(ctx._h, C.byref(camera), C.byref(options), C.byref(sampling),
+                                                            C.byref(adaptive)))
         ctx._session = self
 
     def _live(self):
@@ -551,7 +602,8 @@ class Progressive:
         return self._ctx._h
 
     def step(self, n: int) -> dict:
-        """Renders n more samples per pixel; returns this step's stats (with rays_diffuse and samples)."""
+        """Renders n more samples per pixel (n passes); returns this step's stats (with rays_diffuse and samples), and
+        active_pixels and pixel_samples of the session after it."""
         if n < 0:
             raise CrtError("n must not be negative")
         st = Stats()
@@ -559,7 +611,28 @@ class Progressive:
         self.samples += int(n)
         d = st.as_dict()
         d.update(self._ctx.sampling_stats())
+        pr = self.progress()
+        d["active_pixels"], d["pixel_samples"] = pr["active_pixels"], pr["pixel_samples"]
         return d
+
+    def progress(self) -> dict:
+        """{'passes', 'covered_pixels', 'active_pixels', 'pixel_samples'} (crtb200_accum_progress)."""
+        pr = AccumProgress()
+        _check_core(core().crtb200_accum_progress(self._live(), C.byref(pr)))
+        return {k: getattr(pr, k) for k in ("passes", "covered_pixels", "active_pixels", "pixel_samples")}
+
+    def counts(self) -> np.ndarray:
+        """Per-pixel sample counts n_p (HxW uint32, 0 outside the rects; crtb200_accum_counts)."""
+        counts = np.zeros((self._ctx.height, self._ctx.width), np.uint32)
+        _check_core(core().crtb200_accum_counts(self._live(), counts.ctypes.data))
+        return counts
+
+    def run(self, passes_per_step: int = 8, max_steps: Optional[int] = None) -> list:
+        """Steps until no pixel is active (at most max_steps steps); returns the steps' stats."""
+        out = []
+        while self.progress()["active_pixels"] and (max_steps is None or len(out) < max_steps):
+            out.append(self.step(passes_per_step))
+        return out
 
     def read(self, want_rgb: bool = True, want_rgb8: bool = False, want_hits: bool = False):
         """The image so far: (rgb f32 HxWx3 | None, rgb8 | None, sample 0's hits | None), laid out as Context.render's."""
@@ -573,28 +646,34 @@ class Progressive:
         return rgb, rgb8, hits
 
     def arrays(self) -> dict:
-        """The accumulator: 'sum' and 'sumsq' (HxWx3 f32, 0 outside the rects), 'hit0' (sample 0's hits), 'samples'."""
+        """The accumulator: 'sum' and 'sumsq' (HxWx3 f32, 0 outside the rects), 'hit0' (sample 0's hits), 'samples'
+        (passes) and 'counts' (per-pixel n_p, HxW uint32)."""
         h, w = self._ctx.height, self._ctx.width
         s = np.zeros((h, w, 3), np.float32)
         q = np.zeros((h, w, 3), np.float32)
         hit0 = np.zeros((h, w), HIT_DTYPE)
         n = C.c_uint32(0)
         _check_core(core().crtb200_accum_save(self._live(), s.ctypes.data, q.ctypes.data, hit0.ctypes.data, C.byref(n)))
-        return {"sum": s, "sumsq": q, "hit0": hit0, "samples": np.uint32(n.value)}
+        return {"sum": s, "sumsq": q, "hit0": hit0, "samples": np.uint32(n.value), "counts": self.counts()}
 
     def std_error(self) -> np.ndarray:
-        """Per-pixel, per-channel standard error of the mean, in float64: sqrt(max(0, (Q - S^2 / n) / (n - 1)) / n);
-        NaN below 2 samples.  An estimate of the noise left, not part of the bit-exact contract."""
+        """Per-pixel, per-channel standard error of the mean, in float64: sqrt(max(0, (Q - S^2 / n) / (n - 1)) / n)
+        with the pixel's own count n = n_p (a plain session: its samples, outside the rects too); NaN below 2 samples.
+        An estimate of the noise left, not part of the bit-exact contract."""
         a = self.arrays()
-        n = int(a["samples"])
-        if n < 2:
-            return np.full(a["sum"].shape, np.nan)
+        n = (a["counts"] if self.adaptive is not None else np.full(a["counts"].shape, a["samples"])).astype(np.float64)[..., None]
         s, q = a["sum"].astype(np.float64), a["sumsq"].astype(np.float64)
-        return np.sqrt(np.maximum(0.0, (q - s * s / n) / (n - 1)) / n)
+        with np.errstate(divide="ignore", invalid="ignore"):
+            se = np.sqrt(np.maximum(0.0, (q - s * s / n) / (n - 1)) / n)
+        return np.where(n < 2, np.nan, se)
 
     def save(self, path: str) -> None:
-        """Writes the accumulator and the session's parameters to an .npz file (Context.resume reads it)."""
-        np.savez(path, **self.arrays(), **self._params)
+        """Writes the accumulator and the session's parameters to an .npz file (Context.resume reads it).  A plain
+        session's file has no counts, as before adaptive sessions existed."""
+        a = self.arrays()
+        if self.adaptive is None:
+            del a["counts"]
+        np.savez(path, **a, **self._params)
 
     def close(self) -> None:
         """Ends the session and frees its device memory (crtb200_accum_end)."""

@@ -49,6 +49,9 @@ struct Frame {
   uint32_t sample, spp;               // sample pass of this launch, samples per pixel
   uint32_t seed, frame_index;         // Philox key
   float mc_bias;                      // MONTE_CARLO_BIAS: diffuse ray origin = P + N * mc_bias
+  // adaptive session passes (DESIGN.md 3.10.2): level-0 slot j holds the ray of shard item list[j], j < *n_list (both
+  // written on the device by k_adapt_compact); null in every other launch
+  const uint32_t *list, *n_list;
 };
 
 struct Levels {
@@ -111,7 +114,14 @@ CRT_DI uint32_t warp_alloc(uint32_t *counter, uint32_t n) {
 }
 
 // level-0 work item -> pixel.  Items are numbered tile-major (8x4 tiles) so a warp starts on one coherent tile.
+// LIST: the caller may run in an adaptive pass (GI level-0 kernels), where item_begin + j stands for shard item list[j].
+template <bool LIST = false>
 CRT_DI bool item_pixel(const Frame &fr, const DScene &sc, uint32_t item, uint32_t &row, uint32_t &col) {
+  if (LIST && fr.list) {
+    const uint32_t j = item - fr.item_begin;
+    if (j >= *fr.n_list) return false;
+    item = fr.list[j];
+  }
   const uint32_t local_tile = item >> 5, l = item & 31u;
   const unsigned long long gt = (unsigned long long)local_tile * fr.shard_count + fr.shard_index;
   if (gt >= fr.n_tiles) return false;
@@ -122,6 +132,10 @@ CRT_DI bool item_pixel(const Frame &fr, const DScene &sc, uint32_t item, uint32_
   if (fr.mask && !fr.mask[(size_t)row * sc.width + col]) return false;
   return true;
 }
+
+// level-0 slots of this chunk's launches: the device count of an adaptive pass, else every item of the chunk
+template <bool LIST>
+CRT_DI uint32_t level0_items(const Frame &fr) { return (LIST && fr.list) ? *fr.n_list : fr.n_items0; }
 
 // ------------------------------------------------------------------------------------------------------------
 // MODE 2 building blocks: warp-cooperative triangle phase.
@@ -372,7 +386,7 @@ __global__ void __launch_bounds__(CRT_TRAV_BLOCK, PRIMARY ? CRT_TRAV_MIN_BLOCKS 
   static_assert(MODE == 2, "only loop mode 2 is implemented");
   __shared__ WarpShare s_ws[CRT_TRAV_BLOCK / 32];
   WarpShare *ws = &s_ws[threadIdx.x >> 5];
-  const uint32_t total = PRIMARY ? fr.n_items0 : lv.counts[level];
+  const uint32_t total = PRIMARY ? level0_items<JITTER>(fr) : lv.counts[level];
   const uint32_t node_base = lv.offset[level];
   const uint32_t lane = lane_id();
   const uint32_t tail_start = COUNT ? CRT_INVALID : tail_policy(lv, total, false);
@@ -409,7 +423,7 @@ __global__ void __launch_bounds__(CRT_TRAV_BLOCK, PRIMARY ? CRT_TRAV_MIN_BLOCKS 
         bool valid = true;
         if (PRIMARY) {
           uint32_t row, col;
-          valid = item_pixel(fr, sc, fr.item_begin + i, row, col);
+          valid = item_pixel<JITTER>(fr, sc, fr.item_begin + i, row, col);
           if (valid) {
             if (JITTER)
               jittered_primary_ray(fr, sc.width, sc.height, row, col, ray.o, ray.d);
@@ -566,7 +580,7 @@ static __device__ __noinline__ void spawn_diffuse(const Frame &fr, const Levels 
 // ray_d.w, and every diffuse hit also spawns G diffuse children (COMB_GI).  GI = false is the unsampled kernel.
 template <bool GI>
 __global__ void __launch_bounds__(256) k_shade(const DScene sc, const Frame fr, const Levels lv, const uint32_t level) {
-  const uint32_t total = (level == 0) ? fr.n_items0 : lv.counts[level];
+  const uint32_t total = (level == 0) ? level0_items<GI>(fr) : lv.counts[level];
   const uint32_t node_base = lv.offset[level];
   const uint32_t rounded = (total + 31u) & ~31u;
   uint32_t n_refl = 0, n_refr = 0, n_prim = 0, n_diff = 0;
@@ -578,7 +592,7 @@ __global__ void __launch_bounds__(256) k_shade(const DScene sc, const Frame fr, 
     if (valid) {
       if (level == 0) {
         uint32_t row, col;
-        valid = item_pixel(fr, sc, fr.item_begin + i, row, col);
+        valid = item_pixel<GI>(fr, sc, fr.item_begin + i, row, col);
         if (valid) {
           if (GI) {
             key = jittered_primary_ray(fr, sc.width, sc.height, row, col, o, d);
@@ -1111,7 +1125,7 @@ __global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_co
           shadow_ray_setup(sc, fr, mk(q0.x, q0.y, q0.z), mk(q1.x, q1.y, q1.z), light, ray, dist, contrib);
         } else if (PRIMARY) {
           uint32_t row, col;
-          item_pixel(fr, sc, fr.item_begin + (id - lv.offset[0]), row, col);  // valid: the main kernel started this ray
+          item_pixel<true>(fr, sc, fr.item_begin + (id - lv.offset[0]), row, col);  // valid: the main kernel started this ray
           if (fr.gi)
             jittered_primary_ray(fr, sc.width, sc.height, row, col, ray.o, ray.d);
           else
@@ -1369,13 +1383,13 @@ __global__ void __launch_bounds__(256) k_accumulate(const DScene sc, const Frame
 //                color[node], base from the diffuse item (sampling contract, DESIGN.md 3.10)
 template <bool GI>
 __global__ void __launch_bounds__(256) k_resolve(const DScene sc, const Frame fr, const Levels lv, const uint32_t level) {
-  const uint32_t total = (level == 0) ? fr.n_items0 : lv.counts[level];
+  const uint32_t total = (level == 0) ? level0_items<GI>(fr) : lv.counts[level];
   const uint32_t node_base = lv.offset[level];
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
     const uint32_t node = node_base + i;
     if (level == 0) {
       uint32_t row, col;
-      if (!item_pixel(fr, sc, fr.item_begin + i, row, col)) continue;
+      if (!item_pixel<GI>(fr, sc, fr.item_begin + i, row, col)) continue;
     }
     const uint4 cb = lv.comb[node];
     if (cb.x == COMB_FINAL) continue;
@@ -1638,6 +1652,129 @@ __global__ void __launch_bounds__(256) k_accum_load(const DScene sc, const Frame
       continue;
     }
     hit0[k] = make_uint2(tri, __float_as_uint(r.t));
+  }
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// Adaptive sessions (crtb200_accum_begin_adaptive, DESIGN.md 3.10.2).  Same accumulator; its unused w lanes hold the
+// pixel's sample count n_p (S.w, as uint32 bits) and its active flag (Q.w: 1 = still sampling, 0 = stopped or not
+// covered).  A stopped pixel never starts again, so an active pixel has taken exactly the samples 0 .. passes - 1.
+// ------------------------------------------------------------------------------------------------------------
+struct AdaptParams {
+  uint32_t min_samples, max_samples;
+  float abs_error, rel_error;
+};
+
+// Per pass and chunk: the shard items still sampling, into list[0 .. *n_list) (*n_list zeroed before).  One warp per
+// 8x4 tile, one ballot and one atomicAdd, so a tile's active pixels stay adjacent and a level-0 warp starts coherent.
+// The order of tiles in the list varies from run to run; nothing depends on it (path keys follow the ray's place in
+// its tree, DESIGN.md 3.10).
+__global__ void __launch_bounds__(256) k_adapt_compact(const Frame fr, const float4 *__restrict__ sumsq,
+                                                      uint32_t *__restrict__ list, uint32_t *__restrict__ n_list) {
+  const uint32_t lane = lane_id(), warps = gridDim.x * (blockDim.x >> 5);
+  for (uint32_t t = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); 32u * t < fr.n_items0; t += warps) {
+    const uint32_t i = 32u * t + lane;
+    const bool active = i < fr.n_items0 && sumsq[fr.item_begin + i].w != 0.f;
+    const uint32_t ball = __ballot_sync(CRT_FULL_MASK, active);
+    if (!ball) continue;
+    uint32_t base = 0;
+    if (lane == 0) base = atomicAdd(n_list, (uint32_t)__popc(ball));
+    base = __shfl_sync(CRT_FULL_MASK, base, 0);
+    if (active) list[base + __popc(ball & lanemask_lt())] = fr.item_begin + i;
+  }
+}
+
+// One adaptive pass, in place of k_accum_step: S += c, Q += c c, n_p += 1 at shard item list[j], the hit at sample 0,
+// then the stop rule (crt_s_adapt_stop) clears the active flag.  Counts the pass's shadow rays as k_accum_step does,
+// its pixel-samples into stats[42] and the pixels it stopped into stats[43].
+__global__ void __launch_bounds__(256) k_adapt_step(const DScene sc, const Frame fr, const Levels lv, const AdaptParams ap,
+                                                   float4 *__restrict__ sum, float4 *__restrict__ sumsq,
+                                                   uint2 *__restrict__ hit0) {
+  const uint32_t n_act = *fr.n_list;
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    atomicAdd(&lv.stats[1], (unsigned long long)lv.counts[CRT_MAX_LEVELS] * sc.n_lights);
+    atomicAdd(&lv.stats[42], (unsigned long long)n_act);
+  }
+  const uint32_t stride = gridDim.x * blockDim.x;
+  for (uint32_t base = blockIdx.x * blockDim.x + (threadIdx.x & ~31u); base < n_act; base += stride) {
+    const uint32_t j = base + lane_id();
+    bool stop = false;
+    if (j < n_act) {
+      const uint32_t node = lv.offset[0] + j, k = fr.list[j];
+      const float4 c = lv.color[node], s = sum[k], q = sumsq[k];
+      const V3 a = vadd(mk(s.x, s.y, s.z), mk(c.x, c.y, c.z));
+      const V3 b = vadd(mk(q.x, q.y, q.z), mk(fmul(c.x, c.x), fmul(c.y, c.y), fmul(c.z, c.z)));
+      const uint32_t n = __float_as_uint(s.w) + 1u;
+      const float S[3] = {a.x, a.y, a.z}, Q[3] = {b.x, b.y, b.z};
+      stop = crt_s_adapt_stop(n, S, Q, ap.min_samples, ap.max_samples, ap.abs_error, ap.rel_error) != 0;
+      sum[k] = make_float4(a.x, a.y, a.z, __uint_as_float(n));
+      sumsq[k] = make_float4(b.x, b.y, b.z, stop ? 0.f : 1.f);
+      if (fr.sample == 0) hit0[k] = make_uint2(lv.hit_tri[node], __float_as_uint(lv.hit_t[node]));
+    }
+    const uint32_t stopped = __popc(__ballot_sync(CRT_FULL_MASK, stop));
+    if (lane_id() == 0 && stopped) atomicAdd(&lv.stats[43], (unsigned long long)stopped);
+  }
+}
+
+// Read: S / float(n_p) and the kept hit into the level-0 slots, for k_store (k_accum_read with the pixel's own count)
+__global__ void __launch_bounds__(256) k_adapt_read(const Frame fr, const Levels lv, const float4 *__restrict__ sum,
+                                                   const uint2 *__restrict__ hit0) {
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x) {
+    const uint32_t node = lv.offset[0] + i, k = fr.item_begin + i;
+    const float4 s = sum[k];
+    const uint2 h = hit0[k];
+    const float n = (float)__float_as_uint(s.w);
+    lv.color[node] = make_float4(fdiv(s.x, n), fdiv(s.y, n), fdiv(s.z, n), 0.f);
+    lv.hit_tri[node] = h.x;
+    lv.hit_t[node] = __uint_as_float(h.y);
+  }
+}
+
+// Counts and flags of the covered pixels after begin (counts_in null, passes 0) or a load (behind k_accum_load, which
+// zeroes the w lanes).  counts_in: H*W frame-layout counts, or null for n_p = passes everywhere.  A pixel is active iff
+// n_p == passes and the rule does not stop it at n_p; a count above passes, or 0 while passes > 0, sets *bad.
+// tot[0..2] += covered pixels, active pixels, sum of n_p.
+__global__ void __launch_bounds__(256) k_adapt_counts(const DScene sc, const Frame fr, const uint32_t *__restrict__ counts_in,
+                                                     uint32_t passes, const AdaptParams ap, float4 *__restrict__ sum,
+                                                     float4 *__restrict__ sumsq, uint32_t *__restrict__ bad,
+                                                     unsigned long long *__restrict__ tot) {
+  uint32_t covered = 0, active = 0;
+  unsigned long long samples = 0;
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x) {
+    uint32_t row, col;
+    if (!item_pixel(fr, sc, fr.item_begin + i, row, col)) continue;
+    const uint32_t k = fr.item_begin + i;
+    const uint32_t n = counts_in ? counts_in[(size_t)row * sc.width + col] : passes;
+    if (n > passes || (n == 0 && passes > 0)) {
+      *bad = 1u;
+      continue;
+    }
+    const float4 s = sum[k], q = sumsq[k];
+    const float S[3] = {s.x, s.y, s.z}, Q[3] = {q.x, q.y, q.z};
+    const bool act = n == passes && !crt_s_adapt_stop(n, S, Q, ap.min_samples, ap.max_samples, ap.abs_error, ap.rel_error);
+    sum[k].w = __uint_as_float(n);
+    sumsq[k].w = act ? 1.f : 0.f;
+    covered++;
+    active += act ? 1u : 0u;
+    samples += n;
+  }
+  covered = __reduce_add_sync(CRT_FULL_MASK, covered);
+  active = __reduce_add_sync(CRT_FULL_MASK, active);
+  for (int d = 16; d > 0; d >>= 1) samples += __shfl_xor_sync(CRT_FULL_MASK, samples, d);
+  if (lane_id() == 0 && covered) {
+    atomicAdd(&tot[0], (unsigned long long)covered);
+    atomicAdd(&tot[1], (unsigned long long)active);
+    atomicAdd(&tot[2], samples);
+  }
+}
+
+// Save of the counts map: n_p of the covered pixels into H*W frame-layout counts (the caller zeroes the rest)
+__global__ void __launch_bounds__(256) k_adapt_save(const DScene sc, const Frame fr, const float4 *__restrict__ sum,
+                                                   uint32_t *__restrict__ counts_out) {
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x) {
+    uint32_t row, col;
+    if (!item_pixel(fr, sc, fr.item_begin + i, row, col)) continue;
+    counts_out[(size_t)row * sc.width + col] = __float_as_uint(sum[fr.item_begin + i].w);
   }
 }
 

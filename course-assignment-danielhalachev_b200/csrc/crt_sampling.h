@@ -127,4 +127,27 @@ CRT_S_HD void crt_s_diffuse_dir(uint32_t seed, uint32_t frame, uint32_t p, uint3
   crt_s_normalize(&d[0], &d[1], &d[2]);
   crt_s_normalize(&d[0], &d[1], &d[2]);
 }
+
+/* Stop rule of adaptive sessions (DESIGN.md section 3.10.2), evaluated after a pixel's n-th sample with its running
+ * sums S, Q (per channel, in sample order), in this order:
+ *   nf = (float)n ; m_c = S_c / nf ; v_c = (Q_c - S_c * m_c) / (nf - 1) ; v_c = (v_c > 0) ? v_c : 0
+ *   e_c = sqrt(v_c / nf) ; tol_c = abs_error + rel_error * fabsf(m_c)
+ *   stop  iff  n >= max_samples  ||  (n >= min_samples && e_0 <= tol_0 && e_1 <= tol_1 && e_2 <= tol_2)
+ * min_samples >= 2, so nf - 1 >= 1.  A NaN mean makes tol_c NaN and every comparison false: a pixel with a NaN sample
+ * never stops early and samples up to max_samples. */
+CRT_S_HD int crt_s_adapt_stop(uint32_t n, const float S[3], const float Q[3], uint32_t min_samples, uint32_t max_samples,
+                              float abs_error, float rel_error) {
+  if (n >= max_samples) return 1;
+  if (n < min_samples) return 0;
+  const float nf = (float)n;
+  for (int c = 0; c < 3; c++) {
+    const float m = CRT_S_DIV(S[c], nf);
+    float v = CRT_S_DIV(CRT_S_SUB(Q[c], CRT_S_MUL(S[c], m)), CRT_S_SUB(nf, 1.0f));
+    v = (v > 0.0f) ? v : 0.0f;
+    const float e = CRT_S_SQRT(CRT_S_DIV(v, nf));
+    const float tol = CRT_S_ADD(abs_error, CRT_S_MUL(rel_error, fabsf(m)));
+    if (!(e <= tol)) return 0;
+  }
+  return 1;
+}
 #endif /* CRT_SAMPLING_H */

@@ -199,6 +199,7 @@ struct crtb200_ctx {
     DevBuf<uint4> ovf;          // walks handed off to k_coop (3 x uint4 per record)
     DevBuf<float4> acc;         // GI frames: per level-0 item of the chunk, the running sample sum (k_sample_acc)
     DevBuf<uint2> hit0;         //            ... and sample 0's primary hit
+    DevBuf<uint32_t> alist, acount;  // adaptive passes: the chunk's active shard items and their count (k_adapt_compact)
     uint32_t *work = nullptr;   // into ctl
     cudaStream_t stream = nullptr;
     cudaEvent_t done = nullptr;
@@ -208,6 +209,7 @@ struct crtb200_ctx {
     void release() {
       ray_o.release(); ray_d.release(); color.release(); dq.release(); hit_tri.release(); ctl.release();
       hit_t.release(); comb.release(); vis.release(); ovf.release(); acc.release(); hit0.release();
+      alist.release(); acount.release();
     }
   };
   std::vector<QueueSet> sets;
@@ -251,6 +253,12 @@ struct crtb200_ctx {
   uint32_t acc_done = 0;           // samples in the accumulator
   DevBuf<float4> acc_sum, acc_sumsq;  // S and Q
   DevBuf<uint2> acc_hit;              // sample 0's primary hit {global triangle, bits(t)}
+  // adaptive session (crtb200_accum_begin_adaptive, DESIGN.md 3.10.2): the stop rule's parameters, and totals kept on
+  // the host from each step's counters
+  bool acc_adaptive = false;
+  AdaptParams acc_ap{};
+  uint64_t acc_covered = 0, acc_active_px = 0, acc_px_samples = 0;
+  uint64_t last_px_samples = 0, last_stopped = 0;  // of the last adaptive step (stats[42], stats[43])
 
   // multi-GPU (crtb200_create_multi): this context is the primary (device_ids[0]).  A frame's 8x4-pixel tiles are dealt
   // round-robin over primary + peers (scene replicated); every GPU's k_store writes its pixels STRAIGHT into the
@@ -633,7 +641,9 @@ static int upload_one(crtb200_ctx *c, const crtb200_scene *s);
 // ends the progressive session of a context and frees its accumulators on every GPU
 static void accum_release(crtb200_ctx *c) {
   c->acc_active = false;
+  c->acc_adaptive = false;
   c->acc_done = 0;
+  c->acc_covered = c->acc_active_px = c->acc_px_samples = 0;
   c->acc_rects.clear();
   for (size_t i = 0; i <= c->peers.size(); i++) {
     crtb200_ctx *x = i ? c->peers[i - 1] : c;
@@ -1011,6 +1021,18 @@ static int plan_queues(crtb200_ctx *c, uint32_t shard_items, uint32_t max_depth,
 
 // Pixel coverage of the rectangle list; the mask is only needed when the rectangles do not tile the image exactly
 // (SURVEY App. B-1: the reference then leaves pixels unrendered).
+// per-pixel coverage of a rect list (m: W*H bytes, 1 = covered) and the number of covered pixels
+static size_t rect_coverage(uint32_t W, uint32_t H, const std::vector<crtb200_rect> &rects, std::vector<uint8_t> &m) {
+  m.assign((size_t)W * H, 0);
+  for (const auto &r : rects) {
+    const uint32_t r1 = std::min<uint64_t>(H, (uint64_t)r.row + r.height), c1 = std::min<uint64_t>(W, (uint64_t)r.col + r.width);
+    for (uint32_t y = r.row; y < r1; y++) std::memset(&m[(size_t)y * W + r.col], 1, r.col < c1 ? c1 - r.col : 0);
+  }
+  size_t covered = 0;
+  for (uint8_t v : m) covered += v;
+  return covered;
+}
+
 static int plan_mask(crtb200_ctx *c, const crtb200_options *o) {
   const uint32_t W = c->sc.width, H = c->sc.height;
   std::vector<crtb200_rect> rects(o->rects, o->rects + o->n_rects);
@@ -1020,14 +1042,8 @@ static int plan_mask(crtb200_ctx *c, const crtb200_options *o) {
   c->mask_rects = rects;
   c->mask_needed = false;
   if (!rects.empty()) {
-    std::vector<uint8_t> m((size_t)W * H, 0);
-    for (const auto &r : rects) {
-      const uint32_t r1 = std::min<uint64_t>(H, (uint64_t)r.row + r.height), c1 = std::min<uint64_t>(W, (uint64_t)r.col + r.width);
-      for (uint32_t y = r.row; y < r1; y++) std::memset(&m[(size_t)y * W + r.col], 1, r.col < c1 ? c1 - r.col : 0);
-    }
-    size_t covered = 0;
-    for (uint8_t v : m) covered += v;
-    if (covered != m.size()) {
+    std::vector<uint8_t> m;
+    if (rect_coverage(W, H, rects, m) != m.size()) {
       c->mask_needed = true;
       CUDA_TRY(c->mask.ensure(m.size()));
       CUDA_TRY(cudaMemcpy(c->mask.p, m.data(), m.size(), cudaMemcpyHostToDevice));
@@ -1140,11 +1156,18 @@ struct HostOut {
 // through k_store; SAVE / LOAD move it to / from frame-layout arrays in the primary's memory (peer-mapped on the other
 // GPUs of a multi-GPU context, like k_store's frame).  No pass but STEP runs a sample.
 struct AccumPass {
-  enum Mode { STEP, READ, SAVE, LOAD } mode;
+  enum Mode { STEP, READ, SAVE, LOAD, COUNTS } mode;
   uint32_t s0, n;
   float *px_sum, *px_sumsq;
   HitRec *px_hit;
-  uint32_t *bad;  // LOAD: set when a hit record names no triangle of the scene
+  uint32_t *bad;  // LOAD: set when a hit record names no triangle of the scene (or, adaptive, a count is out of range)
+  // adaptive sessions (DESIGN.md 3.10.2): STEP compacts the active pixels before each sample and runs k_adapt_step;
+  // READ divides by each pixel's own count; SAVE also writes px_counts (if not null); COUNTS sets the counts (px_counts,
+  // null: every count is s0) and the flags, and adds covered pixels, active pixels and pixel-samples into tot[0..2].
+  bool adaptive;
+  AdaptParams ap;
+  uint32_t *px_counts;
+  unsigned long long *tot;
 };
 
 // Enqueue one frame on `st`.  d_rgb / d_rgb8 / d_hits / d_slab are device pointers (any may be null).
@@ -1240,9 +1263,23 @@ static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb20
       CUDA_TRY(q.acc.ensure(c->cap_items));
       CUDA_TRY(q.hit0.ensure(c->cap_items));
     }
+    const bool adapt_step = acc && acc->adaptive && acc->mode == AccumPass::STEP;
+    if (adapt_step) {
+      CUDA_TRY(q.alist.ensure(c->cap_items));
+      CUDA_TRY(q.acount.ensure(1));
+    }
     for (uint32_t s = s_begin; s < s_end; s++) {
       fr.sample = s;
       CUDA_TRY(cudaMemsetAsync(q.ctl.p, 0, q.ctl.n * sizeof(uint32_t), qs));
+      if (adapt_step) {
+        // level 0 of this pass runs over the pixels still sampling; the host keeps n_items0 as the bound
+        fr.list = fr.n_list = nullptr;
+        CUDA_TRY(cudaMemsetAsync(q.acount.p, 0, sizeof(uint32_t), qs));
+        k_adapt_compact<<<grid_simple, 256, 0, qs>>>(fr, c->acc_sumsq.p, q.alist.p, q.acount.p);
+        launches++;
+        fr.list = q.alist.p;
+        fr.n_list = q.acount.p;
+      }
       q.lv.tail_iters = handoff ? (uint32_t)(c->tail_iters + 1) : 0u;
       q.lv.skip_zero_terms = (o->traversal == 0 && o->count_work != 1) ? 1u : 0u;
       q.lv.tail_start = (uint32_t)c->tail_start;
@@ -1317,7 +1354,10 @@ static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb20
           k_resolve<false><<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, l);
         launches++;
       }
-      if (acc) {
+      if (adapt_step) {
+        k_adapt_step<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, acc->ap, c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p);
+        launches++;
+      } else if (acc) {
         k_accum_step<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p);
         launches++;
       } else if (gi) {
@@ -1325,17 +1365,29 @@ static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb20
         launches++;
       }
     }
+    fr.list = fr.n_list = nullptr;
     if (acc && acc->mode == AccumPass::READ) {
       CUDA_TRY(cudaMemsetAsync(q.ctl.p, 0, q.ctl.n * sizeof(uint32_t), qs));  // k_store then counts no shadow rays
-      k_accum_read<<<grid_simple, 256, 0, qs>>>(fr, q.lv, c->acc_sum.p, c->acc_hit.p, acc->s0);
+      if (acc->adaptive)
+        k_adapt_read<<<grid_simple, 256, 0, qs>>>(fr, q.lv, c->acc_sum.p, c->acc_hit.p);
+      else
+        k_accum_read<<<grid_simple, 256, 0, qs>>>(fr, q.lv, c->acc_sum.p, c->acc_hit.p, acc->s0);
       launches++;
     } else if (acc && acc->mode == AccumPass::SAVE) {
       k_accum_save<<<grid_simple, 256, 0, qs>>>(c->sc, fr, c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p, acc->px_sum,
                                                 acc->px_sumsq, acc->px_hit);
       launches++;
+      if (acc->px_counts) {
+        k_adapt_save<<<grid_simple, 256, 0, qs>>>(c->sc, fr, c->acc_sum.p, acc->px_counts);
+        launches++;
+      }
     } else if (acc && acc->mode == AccumPass::LOAD) {
       k_accum_load<<<grid_simple, 256, 0, qs>>>(c->sc, fr, acc->px_sum, acc->px_sumsq, acc->px_hit, c->n_triangles,
                                                 c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p, acc->bad);
+      launches++;
+    } else if (acc && acc->mode == AccumPass::COUNTS) {
+      k_adapt_counts<<<grid_simple, 256, 0, qs>>>(c->sc, fr, acc->px_counts, acc->s0, acc->ap, c->acc_sum.p, c->acc_sumsq.p,
+                                                  acc->bad, acc->tot);
       launches++;
     }
     if (!acc || acc->mode == AccumPass::READ) {
@@ -1443,6 +1495,8 @@ static int collect_stats(crtb200_ctx *c, bool timed) {
     c->last.shadow_rays_zero_term += p->last.shadow_rays_zero_term;
     c->last.kernel_launches += p->last.kernel_launches;
     c->last_diffuse += p->last_diffuse;
+    c->last_px_samples += p->last_px_samples;
+    c->last_stopped += p->last_stopped;
   }
   CUDA_TRY(cudaSetDevice(c->device));
   return CRTB200_OK;
@@ -1507,6 +1561,8 @@ static int collect_stats_one(crtb200_ctx *c, bool timed) {
   c->last.handoff_shadow = st[33];
   c->last.shadow_rays_zero_term = st[40];
   c->last_diffuse = st[41];
+  c->last_px_samples = st[42];
+  c->last_stopped = st[43];
 #if CRT_COOP_STATS
   fprintf(stderr, "[coop stats] closest: %llu walks, %llu iterations, %llu box tests, %llu triangle tests | shadow: %llu walks, %llu iterations, %llu box tests, %llu triangle tests\n",
           st[32], st[34], st[35], st[36], st[33], st[37], st[38], st[39]);
@@ -1719,21 +1775,53 @@ static int session_pass(crtb200_ctx *c, const AccumPass &a, float *d_rgb, uint8_
 struct AccumStaging {
   DevBuf<float> sum, sumsq;
   DevBuf<HitRec> hit;
-  DevBuf<uint32_t> bad;
+  DevBuf<uint32_t> bad, counts;
+  DevBuf<unsigned long long> tot;
   ~AccumStaging() {
     sum.release();
     sumsq.release();
     hit.release();
     bad.release();
+    counts.release();
+    tot.release();
   }
 };
 
-int crtb200_accum_begin(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_options *o, const crtb200_sampling *s) {
-  ErrScope scope(c);
+// The session pass that sets an adaptive session's counts and flags: after begin (passes 0) or behind a load's
+// k_accum_load (g.counts empty = passes everywhere).  g.tot (zeroed by the caller) receives the totals the session
+// keeps on the host; g.bad, when allocated, any out-of-range count.
+static int accum_counts_pass(crtb200_ctx *c, uint32_t passes, AccumStaging &g) {
+  const crtb200_stats keep = c->last;
+  const uint32_t keep_samples = c->last_samples;
+  AccumPass a{AccumPass::COUNTS, passes, 0, nullptr, nullptr, nullptr, g.bad.p};
+  a.adaptive = true;
+  a.ap = c->acc_ap;
+  a.px_counts = g.counts.p;
+  a.tot = g.tot.p;
+  const int rc = session_pass(c, a, nullptr, nullptr, nullptr, false);
+  c->last = keep;
+  c->last_samples = keep_samples;
+  if (rc) return rc;
+  unsigned long long tot[3];
+  CUDA_TRY(cudaMemcpyAsync(tot, g.tot.p, sizeof(tot), cudaMemcpyDeviceToHost, c->stream));
+  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  c->acc_covered = tot[0];
+  c->acc_active_px = tot[1];
+  c->acc_px_samples = tot[2];
+  return CRTB200_OK;
+}
+
+// plain (ad == nullptr) or adaptive session begin; the caller holds the ErrScope
+static int accum_begin(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_options *o, const crtb200_sampling *s,
+                       const crtb200_adaptive *ad) {
   if (!c || !cam || !o || !s) return fail(CRTB200_ERR_ARG, "null argument");
   CUDA_TRY(cudaSetDevice(c->device));
   if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
   if (!s->use_gi) return fail(CRTB200_ERR_ARG, "a progressive session needs sampling.use_gi = 1");
+  if (ad && ad->min_samples < 2) return fail(CRTB200_ERR_ARG, "adaptive: min_samples must be at least 2");
+  if (ad && ad->max_samples < ad->min_samples) return fail(CRTB200_ERR_ARG, "adaptive: max_samples < min_samples");
+  if (ad && !(ad->abs_error >= 0.f && ad->rel_error >= 0.f))
+    return fail(CRTB200_ERR_ARG, "adaptive: the error bounds must be >= 0 and not NaN");
   if (s->gi_samples > 1024) return fail(CRTB200_ERR_ARG, "gi_samples must be at most 1024");
   if (o->shard_count > 1 || o->shard_index != 0)
     return fail(CRTB200_ERR_ARG, "progressive sessions are not tile-sharded (several GPUs: crtb200_create_multi)");
@@ -1770,7 +1858,34 @@ int crtb200_accum_begin(crtb200_ctx *c, const crtb200_camera *cam, const crtb200
   }
   CUDA_TRY(cudaSetDevice(c->device));
   c->acc_active = true;
+  std::vector<uint8_t> m;
+  c->acc_covered = c->acc_rects.empty() ? (uint64_t)c->sc.width * c->sc.height
+                                        : rect_coverage(c->sc.width, c->sc.height, c->acc_rects, m);
+  if (!ad) return CRTB200_OK;
+  c->acc_adaptive = true;
+  c->acc_ap = AdaptParams{ad->min_samples, ad->max_samples, ad->abs_error, ad->rel_error};
+  // every covered pixel starts active: the flags are set on the device, shard by shard
+  AccumStaging g;
+  CUDA_TRY(g.tot.ensure(3));
+  CUDA_TRY(cudaMemsetAsync(g.tot.p, 0, 3 * sizeof(unsigned long long), c->stream));
+  const int rc = accum_counts_pass(c, 0, g);
+  if (rc) {
+    accum_release(c);
+    return rc;
+  }
   return CRTB200_OK;
+}
+
+int crtb200_accum_begin(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_options *o, const crtb200_sampling *s) {
+  ErrScope scope(c);
+  return accum_begin(c, cam, o, s, nullptr);
+}
+
+int crtb200_accum_begin_adaptive(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_options *o,
+                                 const crtb200_sampling *s, const crtb200_adaptive *ad) {
+  ErrScope scope(c);
+  if (!ad) return fail(CRTB200_ERR_ARG, "null argument");
+  return accum_begin(c, cam, o, s, ad);
 }
 
 int crtb200_accum_step(crtb200_ctx *c, uint32_t n_samples, crtb200_stats *stats) {
@@ -1781,13 +1896,19 @@ int crtb200_accum_step(crtb200_ctx *c, uint32_t n_samples, crtb200_stats *stats)
   if (n_samples == 0 || (uint64_t)c->acc_done + n_samples > 0xFFFFFFFFull) return fail(CRTB200_ERR_ARG, "n_samples must be at least 1");
   const auto t0 = std::chrono::steady_clock::now();
   c->last = crtb200_stats{};
-  const AccumPass a{AccumPass::STEP, c->acc_done, n_samples, nullptr, nullptr, nullptr, nullptr};
+  AccumPass a{AccumPass::STEP, c->acc_done, n_samples, nullptr, nullptr, nullptr, nullptr};
+  a.adaptive = c->acc_adaptive;
+  a.ap = c->acc_ap;
   int rc = session_pass(c, a, nullptr, nullptr, nullptr, true);
   if (rc) return rc;
   CUDA_TRY(cudaStreamSynchronize(c->stream));
   rc = collect_stats(c, true);
   if (rc) return rc;
   c->acc_done += n_samples;
+  if (c->acc_adaptive) {
+    c->acc_px_samples += c->last_px_samples;
+    c->acc_active_px -= c->last_stopped;
+  }
   c->last.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
   if (stats) *stats = c->last;
   return CRTB200_OK;
@@ -1805,7 +1926,8 @@ int crtb200_accum_read(crtb200_ctx *c, float *rgb_out, uint8_t *rgb8_out, crtb20
   // a read is no render: the last render's statistics stay what they were
   const crtb200_stats keep = c->last;
   const uint32_t keep_samples = c->last_samples;
-  const AccumPass a{AccumPass::READ, c->acc_done, 0, nullptr, nullptr, nullptr, nullptr};
+  AccumPass a{AccumPass::READ, c->acc_done, 0, nullptr, nullptr, nullptr, nullptr};
+  a.adaptive = c->acc_adaptive;
   const int rc = session_pass(c, a, c->frame.p, rgb8_out ? c->frame8.p : nullptr, hits_out ? c->hits.p : nullptr, false);
   c->last = keep;
   c->last_samples = keep_samples;
@@ -1852,11 +1974,13 @@ int crtb200_accum_save(crtb200_ctx *c, float *sum_out, float *sumsq_out, crtb200
   return CRTB200_OK;
 }
 
-int crtb200_accum_load(crtb200_ctx *c, const float *sum, const float *sumsq, const crtb200_hit *hit0, uint32_t samples_done) {
-  ErrScope scope(c);
+// plain or adaptive load (counts: null = samples_done everywhere); the caller holds the ErrScope
+static int accum_load(crtb200_ctx *c, const float *sum, const float *sumsq, const crtb200_hit *hit0, const uint32_t *counts,
+                      uint32_t samples_done) {
   if (!c || !sum || !sumsq || !hit0) return fail(CRTB200_ERR_ARG, "null argument");
   CUDA_TRY(cudaSetDevice(c->device));
   if (!c->acc_active) return fail(CRTB200_ERR_STATE, "no progressive session (crtb200_accum_begin)");
+  if (counts && !c->acc_adaptive) return fail(CRTB200_ERR_ARG, "a counts map can only be loaded into an adaptive session");
   const size_t px = (size_t)c->sc.width * c->sc.height;
   AccumStaging g;
   CUDA_TRY(g.sum.ensure(px * 3));
@@ -1870,7 +1994,7 @@ int crtb200_accum_load(crtb200_ctx *c, const float *sum, const float *sumsq, con
   const crtb200_stats keep = c->last;
   const uint32_t keep_samples = c->last_samples;
   const AccumPass a{AccumPass::LOAD, 0, 0, g.sum.p, g.sumsq.p, g.hit.p, g.bad.p};
-  const int rc = session_pass(c, a, nullptr, nullptr, nullptr, false);
+  int rc = session_pass(c, a, nullptr, nullptr, nullptr, false);
   c->last = keep;
   c->last_samples = keep_samples;
   if (rc) return rc;
@@ -1882,6 +2006,78 @@ int crtb200_accum_load(crtb200_ctx *c, const float *sum, const float *sumsq, con
     return fail(CRTB200_ERR_ARG, "hit records name triangles the uploaded scene does not have; the session has ended");
   }
   c->acc_done = samples_done;
+  if (!c->acc_adaptive) return CRTB200_OK;
+  // the counts and flags, behind k_accum_load (which zeroed them) on the same streams
+  if (counts) {
+    CUDA_TRY(g.counts.ensure(px));
+    CUDA_TRY(cudaMemcpyAsync(g.counts.p, counts, px * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+  }
+  CUDA_TRY(g.tot.ensure(3));
+  CUDA_TRY(cudaMemsetAsync(g.tot.p, 0, 3 * sizeof(unsigned long long), c->stream));
+  rc = accum_counts_pass(c, samples_done, g);
+  if (rc) return rc;
+  CUDA_TRY(cudaMemcpyAsync(&bad, g.bad.p, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  if (bad) {
+    accum_release(c);
+    return fail(CRTB200_ERR_ARG, "a count exceeds passes, or is 0 inside the rects while passes > 0; the session has ended");
+  }
+  return CRTB200_OK;
+}
+
+int crtb200_accum_load(crtb200_ctx *c, const float *sum, const float *sumsq, const crtb200_hit *hit0, uint32_t samples_done) {
+  ErrScope scope(c);
+  return accum_load(c, sum, sumsq, hit0, nullptr, samples_done);
+}
+
+int crtb200_accum_load_counts(crtb200_ctx *c, const float *sum, const float *sumsq, const crtb200_hit *hit0,
+                              const uint32_t *counts, uint32_t passes) {
+  ErrScope scope(c);
+  return accum_load(c, sum, sumsq, hit0, counts, passes);
+}
+
+int crtb200_accum_progress(crtb200_ctx *c, crtb200_progress *p) {
+  ErrScope scope(c);
+  if (!c || !p) return fail(CRTB200_ERR_ARG, "null argument");
+  if (!c->acc_active) return fail(CRTB200_ERR_STATE, "no progressive session (crtb200_accum_begin)");
+  *p = crtb200_progress{};
+  p->passes = c->acc_done;
+  p->covered_pixels = c->acc_covered;
+  p->active_pixels = c->acc_adaptive ? c->acc_active_px : c->acc_covered;
+  p->pixel_samples = c->acc_adaptive ? c->acc_px_samples : c->acc_covered * c->acc_done;
+  return CRTB200_OK;
+}
+
+int crtb200_accum_counts(crtb200_ctx *c, uint32_t *counts_out) {
+  ErrScope scope(c);
+  if (!c || !counts_out) return fail(CRTB200_ERR_ARG, "null argument");
+  CUDA_TRY(cudaSetDevice(c->device));
+  if (!c->acc_active) return fail(CRTB200_ERR_STATE, "no progressive session (crtb200_accum_begin)");
+  const size_t px = (size_t)c->sc.width * c->sc.height;
+  if (!c->acc_adaptive) {  // every covered pixel has taken every pass
+    if (c->acc_rects.empty()) {
+      std::fill(counts_out, counts_out + px, c->acc_done);
+    } else {
+      std::vector<uint8_t> m;
+      rect_coverage(c->sc.width, c->sc.height, c->acc_rects, m);
+      for (size_t i = 0; i < px; i++) counts_out[i] = m[i] ? c->acc_done : 0u;
+    }
+    return CRTB200_OK;
+  }
+  AccumStaging g;
+  CUDA_TRY(g.counts.ensure(px));
+  CUDA_TRY(cudaMemsetAsync(g.counts.p, 0, px * sizeof(uint32_t), c->stream));
+  const crtb200_stats keep = c->last;
+  const uint32_t keep_samples = c->last_samples;
+  AccumPass a{AccumPass::SAVE, c->acc_done, 0, nullptr, nullptr, nullptr, nullptr};
+  a.adaptive = true;
+  a.px_counts = g.counts.p;
+  const int rc = session_pass(c, a, nullptr, nullptr, nullptr, false);
+  c->last = keep;
+  c->last_samples = keep_samples;
+  if (rc) return rc;
+  CUDA_TRY(cudaMemcpyAsync(counts_out, g.counts.p, px * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+  CUDA_TRY(cudaStreamSynchronize(c->stream));
   return CRTB200_OK;
 }
 

@@ -291,6 +291,44 @@ int crtb200_accum_load(crtb200_ctx *ctx, const float *sum, const float *sumsq, c
 /* replaces: nothing in the reference (see above).  Ends the session and frees its accumulators; no-op without one. */
 int crtb200_accum_end(crtb200_ctx *ctx);
 
+/* Adaptive sessions (DESIGN.md 3.10.2): a progressive session in which each pixel stops sampling once its noise is
+ * below a bound and later passes trace only the pixels still sampling.  After its n-th sample a pixel stops iff
+ * n >= max_samples, or n >= min_samples and every channel's standard error of the mean is at most
+ * abs_error + rel_error * |mean| (the rule of crt_s_adapt_stop in csrc/crt_sampling.h).  A stopped pixel never starts
+ * again, so pixel p of a read is bit for bit crtb200_render's pixel p with rays_per_pixel = n_p, its own count. */
+typedef struct crtb200_adaptive {
+  uint32_t min_samples; /* >= 2 */
+  uint32_t max_samples; /* >= min_samples */
+  float abs_error;      /* >= 0 */
+  float rel_error;      /* >= 0 */
+} crtb200_adaptive;
+
+typedef struct crtb200_progress {
+  uint32_t passes;          /* passes run so far (samples of a plain session)                       */
+  uint32_t reserved;
+  uint64_t covered_pixels;  /* pixels inside the session's rects                                      */
+  uint64_t active_pixels;   /* covered pixels still sampling (every covered pixel of a plain session) */
+  uint64_t pixel_samples;   /* sum of the per-pixel sample counts (covered x passes when plain)       */
+} crtb200_progress;
+
+/* replaces: nothing in the reference.  crtb200_accum_begin with a stop rule, fixed for the session's life.  A step of n
+ * runs n passes; pass s renders sample s of every active pixel as a one-shot frame renders it.  CRTB200_ERR_ARG, besides
+ * crtb200_accum_begin's cases, when min_samples < 2, max_samples < min_samples or an error bound is negative or NaN. */
+int crtb200_accum_begin_adaptive(crtb200_ctx *ctx, const crtb200_camera *camera, const crtb200_options *options,
+                                 const crtb200_sampling *sampling, const crtb200_adaptive *adaptive);
+/* replaces: nothing in the reference.  Passes, covered and active pixels and pixel-samples of the session (plain or
+ * adaptive).  CRTB200_ERR_STATE without a session. */
+int crtb200_accum_progress(crtb200_ctx *ctx, crtb200_progress *progress);
+/* replaces: nothing in the reference.  counts_out: H*W per-pixel sample counts n_p, 0 outside the rects.
+ * CRTB200_ERR_STATE without a session. */
+int crtb200_accum_counts(crtb200_ctx *ctx, uint32_t *counts_out);
+/* replaces: nothing in the reference.  crtb200_accum_load of an adaptive session with its counts map (H*W, as
+ * crtb200_accum_counts writes it; NULL = passes everywhere).  A pixel is active iff n_p == passes and the rule does not
+ * stop it at n_p.  CRTB200_ERR_ARG, and the session ends, when a count inside the rects exceeds passes or is 0 while
+ * passes > 0; CRTB200_ERR_ARG when the session is plain and counts is not NULL. */
+int crtb200_accum_load_counts(crtb200_ctx *ctx, const float *sum, const float *sumsq, const crtb200_hit *hit0,
+                              const uint32_t *counts, uint32_t passes);
+
 /* replaces: the data RayTracer keeps in `scene`, `boundingBox`, `accelerationStructure` (RayTracer.h:64-67).
  * Copies + re-lays-out everything to device SoA during the call (host flattener H1). */
 int crtb200_upload_scene(crtb200_ctx *ctx, const crtb200_scene *scene);
