@@ -117,13 +117,13 @@ def test_degenerate_equals_plain(loaded, crt):
 
 
 def _bits(ctx, crt, sf, opt, cfg, steps):
+    """The session's image and arrays, and the walks its steps handed off to k_coop (closest hit)."""
     p = ctx.progressive(sf.camera(), opt, _smp(crt, cfg), _ad(crt, 2, 8))
-    for s in steps:
-        p.step(s)
+    handed_off = sum(p.step(s)["handoff_closest"] for s in steps)
     rgb = p.read()[0]
     a = p.arrays()
     p.close()
-    return rgb, a
+    return rgb, a, handed_off
 
 
 def test_invariance(loaded, crt):
@@ -143,16 +143,23 @@ def test_invariance(loaded, crt):
         variants.append(("traversal 1", _bits(ctx, crt, sf, crt.make_options(max_depth=cfg["depth"], traversal=1), cfg, (3, 5))))
     finally:
         ctx.close()
-    multi = _context(crt, sf, flat, [0, 0, 0])
-    try:
-        variants.append(("Context([0, 0, 0])", _bits(multi, crt, sf, opt, cfg, (3, 5))))
-    finally:
-        multi.close()
+    # forced hand-off: k_coop maps the level-0 slots of handed-off primary walks through the pass's active list
+    forced = []
+    for which, devices in (("default", [0, 0, 0]), ("all", 0), ("mid", 0), ("capped", 0), ("mid", [0, 0, 0])):
+        ctx = _context(crt, sf, flat, devices, which)
+        try:
+            variants.append((f"Context({devices}), hand-off {which}", _bits(ctx, crt, sf, opt, cfg, (3, 5))))
+            if which != "default":
+                forced.append(variants[-1])
+        finally:
+            ctx.close()
     assert len(np.unique(ref[1]["counts"])) >= 3
-    for what, (rgb, a) in variants:
+    for what, (rgb, a, _) in variants:
         assert same_f32(rgb, ref[0]).all(), what
         for k in ("sum", "sumsq", "counts"):
             assert same_f32(a[k].view(np.float32), ref[1][k].view(np.float32)).all(), (what, k)
+    for what, (_, _, handed_off) in forced:
+        assert handed_off > 0, what
 
 
 @pytest.mark.parametrize("devices", [(0, 0), (0, [0, 0, 0]), ([0, 0, 0], 0)], ids=["single", "single_to_multi", "multi_to_single"])

@@ -8,10 +8,15 @@ import os
 import numpy as np
 import pytest
 
+import gi_oracle as gio
 from conftest import PKG, ROOT, SMALL_SCENES, same_f32
+from handoff_contexts import HandoffContexts
 
 pytestmark = pytest.mark.gpu
 GOLDEN = os.path.join(ROOT, "tests", "golden")
+# hw14_small's 20 736 primary rays are more than the "capped" context's k_coop takes in one launch (4 736 walks on a B200:
+# one per resident k_coop warp)
+CAPPED_OVERFLOW = "hw14_small"
 
 
 @pytest.fixture(scope="module")
@@ -234,65 +239,29 @@ def test_production_path_matches_golden(name, gpu, loaded, crt):
     assert [st["rays_primary"], st["rays_shadow"], st["rays_reflection"], st["rays_refraction"]] == list(g["rays"])
 
 
-def _ctx_with_env(built, **env):
-    """A context created under tuning environment variables (crtb200_create reads them once)."""
-    old = {k: os.environ.get(k) for k in env}
-    os.environ.update({k: str(v) for k, v in env.items()})
-    try:
-        return built.Context(0)
-    finally:
-        for k, v in old.items():
-            if v is None:
-                del os.environ[k]
-            else:
-                os.environ[k] = v
-
-
 @pytest.fixture(scope="module")
-def gpu_coop_all(built):
-    """Every walk is handed to k_coop before its first step (a small frame's queue is dry after the first refill, and
-    a threshold of 0 iterations hands off at once): the warp-per-ray walk does ALL the traversal work of the frame."""
-    ctx = _ctx_with_env(built, CRT_TAIL_ITERS=0, CRT_TAIL_START=0, CRT_TAIL_SMALL=100000000, CRT_TAIL_CAP=1000000)
-    yield ctx
-    ctx.close()
+def handoff(built):
+    """Contexts with the tail hand-off forced or off (handoff_contexts.HANDOFF_ENV), created on first use."""
+    hc = HandoffContexts(built)
+    yield hc
+    hc.close()
 
 
-@pytest.fixture(scope="module")
-def gpu_coop_mid(built):
-    """Walks are handed off in mid-flight: whatever has taken 3 node-phase iterations when the queue is dry."""
-    ctx = _ctx_with_env(built, CRT_TAIL_ITERS=3, CRT_TAIL_START=3, CRT_TAIL_SMALL=100000000, CRT_TAIL_CAP=1000000)
-    yield ctx
-    ctx.close()
-
-
-@pytest.fixture(scope="module")
-def gpu_coop_final_only(built):
-    """Every walk handed off, and k_coop's early pass (next to the traversal kernel) switched off: the final pass alone."""
-    ctx = _ctx_with_env(built, CRT_TAIL_ITERS=0, CRT_TAIL_START=0, CRT_TAIL_SMALL=100000000, CRT_TAIL_CAP=1000000, CRT_COOP_EARLY=0)
-    yield ctx
-    ctx.close()
-
-
-@pytest.fixture(scope="module")
-def gpu_no_handoff(built):
-    ctx = _ctx_with_env(built, CRT_TAIL_ITERS=-1)
-    yield ctx
-    ctx.close()
-
-
-@pytest.mark.parametrize("which", ["all", "mid", "final_only", "off"])
+@pytest.mark.parametrize("which", ["all", "mid", "final_only", "off", "capped"])
 @pytest.mark.parametrize("name", list(SMALL_SCENES))
-def test_tail_handoff_matches_golden(name, which, gpu_coop_all, gpu_coop_mid, gpu_coop_final_only, gpu_no_handoff, loaded, crt):
+def test_tail_handoff_matches_golden(name, which, handoff, loaded, crt):
     """k_coop explores a handed-off walk in a different order (a LIFO of subtrees, 32 boxes per iteration); by the nesting
     property the set of tested leaves is the same, and closest-hit candidates are put back into the reference's
     encounter order by their (leaf, reference) key -- so hit ids, t and every pixel stay bit-identical to the
     reference fixtures, with culling (traversal 0) and without (traversal 1 has no hand-off: literal walk).  "all" and "mid"
     run k_coop's early pass next to the traversal kernel plus the final pass behind it (small frames run on one stream),
-    "final_only" the final pass alone."""
-    ctx = {"all": gpu_coop_all, "mid": gpu_coop_mid, "final_only": gpu_coop_final_only, "off": gpu_no_handoff}[which]
+    "final_only" the final pass alone.  "capped" asks to hand off every walk, but k_coop takes one walk per resident warp
+    and launch: the lanes turned away keep walking in the traversal kernel."""
+    ctx = handoff(which)
     sf, flat, rects, n = loaded[name]
     ctx.upload(flat, keepalive=sf)
-    rgb, rgb8, hits, st = ctx.render(sf.camera(), crt.make_options(rects=rects, n_rects=n), want_rgb8=True, want_hits=True)
+    opt = crt.make_options(rects=rects, n_rects=n)
+    rgb, rgb8, hits, st = ctx.render(sf.camera(), opt, want_rgb8=True, want_hits=True)
     g = np.load(os.path.join(GOLDEN, name + ".npz"))
     cov = _covered(sf, rects, n)
     assert np.array_equal(hits["mesh"][cov], g["hits"]["mesh"][cov]) and np.array_equal(hits["triangle"][cov], g["hits"]["triangle"][cov])
@@ -300,13 +269,18 @@ def test_tail_handoff_matches_golden(name, which, gpu_coop_all, gpu_coop_mid, gp
     assert same_f32(hits["t"][h], g["hits"]["t"][h]).all()
     _assert_pixels(name, rgb, g["rgb"], rgb8, g["ppm"])
     assert [st["rays_primary"], st["rays_shadow"], st["rays_reflection"], st["rays_refraction"]] == list(g["rays"])
-    if which in ("all", "final_only") and name not in ("empty_scene",):
+    if which in ("all", "final_only", "capped") and name not in ("empty_scene",):
         assert st["handoff_closest"] > 0  # (warps that fetched their rays before the queue ran dry poll it every 4th round)
     if which == "off":
         assert st["handoff_closest"] == 0 and st["handoff_shadow"] == 0
+    if which == "capped" and name == CAPPED_OVERFLOW:
+        # the capacity is reached: fewer walks are handed off than on the same frame with room for every walk
+        handoff("all").upload(flat, keepalive=sf)
+        _, _, _, st_all = handoff("all").render(sf.camera(), opt)
+        assert st["handoff_closest"] < st_all["handoff_closest"], (st["handoff_closest"], st_all["handoff_closest"])
 
 
-def test_tail_handoff_full_size_equals_literal_walk(gpu, gpu_coop_mid, built):
+def test_tail_handoff_full_size_equals_literal_walk(gpu, handoff, built):
     """1920x1080 room with 196 608-triangle mirror and glass spheres, depth 5 (thousands of long walks on every level):
     default kernels, aggressive mid-flight hand-off and the literal walk must agree bit for bit."""
     import importlib
@@ -315,7 +289,7 @@ def test_tail_handoff_full_size_equals_literal_walk(gpu, gpu_coop_mid, built):
     sf = built.SceneFile(f, folder)
     flat = sf.flatten()
     outs = []
-    for ctx, trav in ((gpu, 1), (gpu, 0), (gpu_coop_mid, 0)):
+    for ctx, trav in ((gpu, 1), (gpu, 0), (handoff("mid"), 0)):
         ctx.upload(flat, keepalive=sf)
         rgb, _, hits, st = ctx.render(sf.camera(), built.make_options(max_depth=depth, traversal=trav), want_hits=True)
         outs.append((rgb, hits, st))
@@ -326,10 +300,11 @@ def test_tail_handoff_full_size_equals_literal_walk(gpu, gpu_coop_mid, built):
         assert outs[0][2]["rays_total"] == outs[k][2]["rays_total"]
 
 
-def test_trees_that_do_not_nest_take_the_literal_walk(gpu, built, scene_dir, ob, crt):
+def test_trees_that_do_not_nest_take_the_literal_walk(gpu, handoff, built, scene_dir, ob, crt):
     """Culling and the order-free walk of k_coop are only equivalent to the reference's walk when every child box lies
     inside its parent's.  A caller may upload any tree through the C ABI: shrink one inner box so its children stick out
-    -> the library must fall back to the literal walk, i.e. still agree with the oracle run on the very same (odd) tree."""
+    -> the library must fall back to the literal walk, i.e. still agree with the oracle run on the very same (odd) tree.
+    GI frames too, even in a context that would hand off every walk."""
     sf = built.SceneFile("hw14_small.crtscene", scene_dir)
     flat = sf.flatten()
     s = flat.contents
@@ -352,6 +327,19 @@ def test_trees_that_do_not_nest_take_the_literal_walk(gpu, built, scene_dir, ob,
     assert a["handoff_closest"] == a["handoff_shadow"] == 0
     assert a["shadow_rays_zero_term"] > 0 and b["shadow_rays_zero_term"] == 0
     assert a["node_tests_shadow"] < b["node_tests_shadow"]
+    ctx = handoff("all")
+    ctx.upload(flat, keepalive=sf)
+    smp = crt.Sampling.make(gi_samples=1, rays_per_pixel=2, seed=11)
+    opt = crt.make_options(max_depth=5)
+    ctx.set_sampling(smp)
+    g_rgb, _, g_hits, g = ctx.render(sf.camera(), opt, want_hits=True)
+    ctx.set_sampling(None)
+    o_rgb, o_hits, o_st = gio.render_sampled(flat, sf.camera(), opt, smp)
+    assert same_f32(g_rgb, o_rgb).all(), f"{(~same_f32(g_rgb, o_rgb)).sum()} components differ"
+    assert np.array_equal(g_hits["mesh"], o_hits["mesh"]) and np.array_equal(g_hits["triangle"], o_hits["triangle"])
+    assert [g[k] for k in ("rays_primary", "rays_shadow", "rays_reflection", "rays_refraction")] == \
+        [o_st[k] for k in ("rays_primary", "rays_shadow", "rays_reflection", "rays_refraction")]
+    assert g["handoff_closest"] == g["handoff_shadow"] == 0
 
 
 def test_multi_gpu_context_matches_single(gpu, built, loaded, crt):

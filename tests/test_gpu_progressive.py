@@ -8,6 +8,7 @@ import pytest
 
 import progressive_oracle as po
 from conftest import SMALL_SCENES, same_f32
+from handoff_contexts import handoff_context
 
 pytestmark = pytest.mark.gpu
 CONFIGS = [dict(G=1, depth=5), dict(G=2, depth=3)]
@@ -45,8 +46,9 @@ def _same_frame(got, want, cov):
     assert same_f32(hits["t"][hit], w_hits["t"][hit]).all()
 
 
-def _context(crt, sf, flat, devices=0):
-    ctx = crt.Context(devices)
+def _context(crt, sf, flat, devices=0, handoff="default"):
+    """A context holding the scene; `handoff` names the tail hand-off setting (handoff_contexts.HANDOFF_ENV)."""
+    ctx = handoff_context(crt, handoff, devices)
     ctx.upload(flat, keepalive=sf)
     return ctx
 
@@ -133,11 +135,12 @@ def test_invariance(loaded, crt):
         variants.append(("traversal 1", _session_bits(ctx, crt, sf, crt.make_options(max_depth=cfg["depth"], traversal=1), cfg)))
     finally:
         ctx.close()
-    multi = _context(crt, sf, flat, [0, 0, 0])
-    try:
-        variants.append(("Context([0, 0, 0])", _session_bits(multi, crt, sf, opt, cfg)))
-    finally:
-        multi.close()
+    for which, devices in (("default", [0, 0, 0]), ("all", 0), ("mid", 0), ("capped", 0), ("mid", [0, 0, 0])):
+        ctx = _context(crt, sf, flat, devices, which)
+        try:
+            variants.append((f"Context({devices}), hand-off {which}", _session_bits(ctx, crt, sf, opt, cfg)))
+        finally:
+            ctx.close()
     for what, (rgb, a) in variants:
         assert same_f32(rgb, ref).all(), what
         for k in ("sum", "sumsq"):
