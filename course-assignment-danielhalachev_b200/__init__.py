@@ -77,6 +77,28 @@ class Scene(C.Structure):
     ]
 
 
+class Trees(C.Structure):
+    """crtb200_trees: the trees of the last crtb200_upload_geometry (crtb200_scene_trees)."""
+    _fields_ = [("n_meshes", C.c_uint32), ("n_mesh_nodes", C.c_uint32), ("n_mesh_leaf_refs", C.c_uint32),
+                ("n_top_nodes", C.c_uint32), ("n_top_leaf_refs", C.c_uint32), ("reserved", C.c_uint32),
+                ("peak_scratch_bytes", C.c_uint64), ("build_ms", C.c_double),
+                ("meshes", C.c_void_p), ("mesh_nodes", C.c_void_p), ("mesh_leaf_refs", C.c_void_p),
+                ("top_nodes", C.c_void_p), ("top_leaf_refs", C.c_void_p)]
+
+
+class SceneLayout(C.Structure):
+    """crtb200_scene_layout: one GPU's device scene state (crtb200_debug_scene_layout)."""
+    _fields_ = [("n_nodes", C.c_uint32), ("n_leaf_refs", C.c_uint32), ("n_top_refs", C.c_uint32), ("n_meshes", C.c_uint32),
+                ("top_begin", C.c_uint32), ("top_end", C.c_uint32), ("nested_ok", C.c_uint32), ("reserved", C.c_uint32),
+                ("nodes", C.c_void_p), ("leaf_refs", C.c_void_p), ("top_refs", C.c_void_p), ("meshes", C.c_void_p)]
+
+
+# numpy views of crtb200_kdnode and crtb200_mesh records
+KDNODE_DTYPE = np.dtype([("box_min", np.float32, 3), ("box_max", np.float32, 3), ("child", np.uint32, 2),
+                         ("leaf_start", np.uint32), ("leaf_count", np.uint32)])
+MESH_DTYPE = np.dtype([(n, np.uint32) for n, _ in Mesh._fields_])
+
+
 class Camera(C.Structure):
     _fields_ = [("position", C.c_float * 3), ("rotation", C.c_float * 9)]
 
@@ -202,6 +224,9 @@ def core() -> C.CDLL:
         lib.crtb200_trace_rays.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]
         lib.crtb200_device_count.argtypes = [C.POINTER(C.c_int)]
         lib.crtb200_debug_powf5.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]
+        lib.crtb200_upload_geometry.argtypes = [C.c_void_p, C.POINTER(Scene)]
+        lib.crtb200_scene_trees.argtypes = [C.c_void_p, C.POINTER(Trees)]
+        lib.crtb200_debug_scene_layout.argtypes = [C.c_void_p, C.c_int, C.POINTER(SceneLayout)]
         lib.crtb200_set_sampling.argtypes = [C.c_void_p, C.POINTER(Sampling)]
         lib.crtb200_last_sampling_stats.argtypes = [C.c_void_p, C.POINTER(SamplingStats)]
         lib.crtb200_accum_begin.argtypes = [C.c_void_p, C.POINTER(Camera), C.POINTER(Options), C.POINTER(Sampling)]
@@ -232,6 +257,7 @@ def front() -> C.CDLL:
         lib.crtfe_scene_free.argtypes = [C.c_void_p]
         lib.crtfe_scene_get_info.argtypes = [C.c_void_p, C.POINTER(SceneInfo)]
         lib.crtfe_scene_flatten.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.POINTER(Scene)), C.POINTER(C.c_double)]
+        lib.crtfe_scene_flatten_geometry.argtypes = [C.c_void_p, C.POINTER(C.POINTER(Scene)), C.POINTER(C.c_double)]
         lib.crtfe_rectangles.argtypes = [C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Rect), C.c_uint32, C.POINTER(C.c_uint32)]
         lib.crtfe_camera_pan.argtypes = [C.POINTER(Camera), C.c_float]
         lib.crtfe_camera_tilt.argtypes = [C.POINTER(Camera), C.c_float]
@@ -280,13 +306,25 @@ class SceneFile:
         self.info = SceneInfo()
         _check_front(front().crtfe_scene_get_info(self._h, C.byref(self.info)))
         self._flat: Optional[C.POINTER(Scene)] = None
+        self._geometry: Optional[C.POINTER(Scene)] = None
         self.build_seconds = 0.0
+        self.geometry_seconds = 0.0
 
     @property
     def handle(self):
         return self._h
 
-    def flatten(self, threads: int = 0) -> "C.POINTER(Scene)":
+    def flatten(self, threads: int = 0, trees: bool = True) -> "C.POINTER(Scene)":
+        """The scene as crtb200_scene arrays, with the host-built KD trees (crtb200_upload_scene), or with trees=False
+        without them (tree counts 0, arrays NULL: Context.upload_geometry builds them on the GPU).  Each is built once."""
+        if not trees:
+            if self._geometry is None:
+                p = C.POINTER(Scene)()
+                sec = C.c_double(0)
+                _check_front(front().crtfe_scene_flatten_geometry(self._h, C.byref(p), C.byref(sec)))
+                self._geometry = p
+                self.geometry_seconds = sec.value
+            return self._geometry
         if self._flat is None:
             p = C.POINTER(Scene)()
             sec = C.c_double(0)
@@ -308,6 +346,7 @@ class SceneFile:
             front().crtfe_scene_free(self._h)
             self._h = C.c_void_p()
             self._flat = None
+            self._geometry = None
 
     def __del__(self):
         try:
@@ -403,6 +442,43 @@ class Context:
         _check_core(core().crtb200_upload_scene(self._h, scene_ptr))
         self.width, self.height = scene_ptr.contents.width, scene_ptr.contents.height
         self._scene_keepalive = keepalive
+
+    def upload_geometry(self, scene_ptr, keepalive=None) -> None:
+        """crtb200_upload_geometry: uploads a scene without trees (SceneFile.flatten(trees=False), or a Scene built from
+        arrays) and builds its KD trees on every GPU of the context; afterwards the context is as upload() of the
+        host-built trees leaves it."""
+        _check_core(core().crtb200_upload_geometry(self._h, scene_ptr))
+        self.width, self.height = scene_ptr.contents.width, scene_ptr.contents.height
+        self._scene_keepalive = keepalive
+
+    def scene_trees(self) -> dict:
+        """The trees the last upload_geometry built, in the reference's numbering (crtb200_scene_trees): 'meshes'
+        (MESH_DTYPE, tree fields filled), 'mesh_nodes' / 'top_nodes' (KDNODE_DTYPE), 'mesh_leaf_refs' (mesh-local
+        triangle indices), 'top_leaf_refs' (mesh indices), 'peak_scratch_bytes' and 'build_ms'."""
+        t = Trees()
+        _check_core(core().crtb200_scene_trees(self._h, C.byref(t)))
+        out = {"meshes": np.zeros(t.n_meshes, MESH_DTYPE), "mesh_nodes": np.zeros(t.n_mesh_nodes, KDNODE_DTYPE),
+               "mesh_leaf_refs": np.zeros(t.n_mesh_leaf_refs, np.uint32), "top_nodes": np.zeros(t.n_top_nodes, KDNODE_DTYPE),
+               "top_leaf_refs": np.zeros(t.n_top_leaf_refs, np.uint32)}
+        for k, a in out.items():
+            setattr(t, k, a.ctypes.data)
+        _check_core(core().crtb200_scene_trees(self._h, C.byref(t)))
+        out["peak_scratch_bytes"], out["build_ms"] = t.peak_scratch_bytes, t.build_ms
+        return out
+
+    def debug_scene_layout(self, device_index: int = 0) -> dict:
+        """One GPU's device scene state (crtb200_debug_scene_layout): 'nodes' (n x 8 uint32: min.xyz, a, max.xyz, b of the
+        visiting-order array), 'leaf_refs', 'top_refs', 'meshes' (n x 5 uint32: node_begin, node_end, material,
+        first_triangle, cull_margin bits), 'top_begin', 'top_end' and 'nested_ok'."""
+        l = SceneLayout()
+        _check_core(core().crtb200_debug_scene_layout(self._h, device_index, C.byref(l)))
+        out = {"nodes": np.zeros((l.n_nodes, 8), np.uint32), "leaf_refs": np.zeros(l.n_leaf_refs, np.uint32),
+               "top_refs": np.zeros(l.n_top_refs, np.uint32), "meshes": np.zeros((l.n_meshes, 5), np.uint32)}
+        for k, a in out.items():
+            setattr(l, k, a.ctypes.data)
+        _check_core(core().crtb200_debug_scene_layout(self._h, device_index, C.byref(l)))
+        out.update(top_begin=l.top_begin, top_end=l.top_end, nested_ok=bool(l.nested_ok))
+        return out
 
     def set_queue_budget(self, nbytes: int) -> None:
         _check_core(core().crtb200_set_queue_budget(self._h, nbytes))

@@ -18,7 +18,10 @@
 #include <string>
 #include <vector>
 
+#include <cub/device/device_scan.cuh>
+
 #include "../../include/crtb200.h"
+#include "crt_build.cuh"
 #include "crt_kernels.cuh"
 
 using namespace crtd;
@@ -171,6 +174,14 @@ struct crtb200_ctx {
   DevBuf<DLight> lights;
   bool has_reflective = false, has_refractive = false;
   uint64_t scene_bytes = 0;
+  uint32_t n_nodes = 0, n_leaf_refs = 0, n_top_refs = 0;  // of the uploaded scene (crtb200_debug_scene_layout)
+  // crtb200_upload_geometry: the trees it built, in the reference's numbering, kept on the first GPU of the context for
+  // crtb200_scene_trees (40 bytes per node and 4 per mesh leaf reference; the top-level references are top_refs)
+  bool trees_built = false;
+  DevBuf<crtb200_kdnode> kd_nodes;
+  DevBuf<uint32_t> kd_refs;
+  std::vector<crtb200_mesh> kd_meshes;
+  crtb200_trees kd_counts{};
 
   // frame
   DevBuf<float> frame;   // persistent colour buffer (RayTracer::colorBuffer, RayTracer.h:69)
@@ -410,6 +421,7 @@ int crtb200_destroy(crtb200_ctx *c) {
   c->texels.release(); c->lights.release(); c->frame.release(); c->frame8.release(); c->hits.release();
   c->mask.release(); c->frame_b.release(); c->frame8_b.release();
   c->acc_sum.release(); c->acc_sumsq.release(); c->acc_hit.release();
+  c->kd_nodes.release(); c->kd_refs.release();
   if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
   for (int k = 0; k < 2; k++) {
     if (c->rendered[k]) cudaEventDestroy(c->rendered[k]);
@@ -673,20 +685,61 @@ static int on_all_devices(crtb200_ctx *c, F0 fn0, F fn) {
   return rc;
 }
 
+static int upload_geometry_one(crtb200_ctx *c, const crtb200_scene *s, bool keep);
+
 extern "C" {
 
 int crtb200_upload_scene(crtb200_ctx *c, const crtb200_scene *s) {
   if (!c || !s) return fail(CRTB200_ERR_ARG, "null argument");
   ErrScope scope(c);
   if (c->acc_active) accum_release(c);  // a new scene ends the progressive session
+  c->trees_built = false;
+  c->kd_nodes.release();
+  c->kd_refs.release();
   if (c->peers.empty()) return upload_one(c, s);
   // scene replicated on every GPU (SURVEY 8(e)); the host relayout runs once per GPU, in parallel
   return on_all_devices(c, [&] { return upload_one(c, s); }, [&](size_t, crtb200_ctx *p) { return upload_one(p, s); });
 }
 
+int crtb200_upload_geometry(crtb200_ctx *c, const crtb200_scene *s) {
+  if (!c || !s) return fail(CRTB200_ERR_ARG, "null argument");
+  ErrScope scope(c);
+  if (s->n_mesh_nodes || s->n_mesh_leaf_refs || s->n_top_nodes || s->n_top_leaf_refs || s->mesh_nodes || s->mesh_leaf_refs ||
+      s->top_nodes || s->top_leaf_refs)
+    return fail(CRTB200_ERR_ARG, "crtb200_upload_geometry builds the trees: the scene's tree counts must be 0 and their arrays NULL");
+  if (c->acc_active) accum_release(c);
+  c->trees_built = false;
+  c->kd_nodes.release();
+  c->kd_refs.release();
+  // one build per GPU, in parallel; only the first GPU keeps the reference-numbered trees for crtb200_scene_trees
+  const int rc = c->peers.empty() ? upload_geometry_one(c, s, true)
+                                  : on_all_devices(c, [&] { return upload_geometry_one(c, s, true); },
+                                                   [&](size_t, crtb200_ctx *p) { return upload_geometry_one(p, s, false); });
+  if (rc) {
+    c->trees_built = false;
+    c->kd_nodes.release();
+    c->kd_refs.release();
+  }
+  return rc;
+}
+
 }  // extern "C"
 
-static int upload_one(crtb200_ctx *c, const crtb200_scene *s) {
+// What both upload paths build on the host from the scene's arrays (everything but the trees), after validating them.
+struct SceneRecords {
+  std::vector<float4> geom;
+  std::vector<uint4> shade;
+  std::vector<float4> vn;
+  std::vector<float2> uv;
+  std::vector<DMaterial> mats;
+  std::vector<DTexture> texs;
+  std::vector<float> texels;
+  std::vector<DLight> lights;
+};
+
+// Validation and host records of the triangles, vertices, materials, textures and lights; `trees`: also check the
+// meshes' node and leaf-reference ranges (crtb200_upload_scene).  Selects the context's device and drops its scene.
+static int pack_records(crtb200_ctx *c, const crtb200_scene *s, bool trees, SceneRecords &r) {
   if (s->abi_version != CRTB200_ABI_VERSION) return fail(CRTB200_ERR_ARG, "crtb200_scene.abi_version mismatch");
   if (s->width == 0 || s->height == 0) return fail(CRTB200_ERR_SCENE, "image size is zero");
   if ((uint64_t)s->width * s->height > 0x7FFFFFFFull / 4) return fail(CRTB200_ERR_SCENE, "image too large");
@@ -700,15 +753,15 @@ static int upload_one(crtb200_ctx *c, const crtb200_scene *s) {
   c->have_scene = false;
 
   // triangles
-  std::vector<float4> geom(3 * (size_t)s->n_triangles);
-  std::vector<uint4> shade(s->n_triangles);
+  r.geom.resize(3 * (size_t)s->n_triangles);
+  r.shade.resize(s->n_triangles);
   std::vector<uint32_t> tri_mesh(s->n_triangles, CRTB200_INVALID);
   for (uint32_t m = 0; m < s->n_meshes; m++) {
     const crtb200_mesh &me = s->meshes[m];
     if ((uint64_t)me.first_triangle + me.n_triangles > s->n_triangles) return fail(CRTB200_ERR_SCENE, "mesh triangle range out of bounds");
     if (me.material >= s->n_materials) return fail(CRTB200_ERR_SCENE, "mesh material index out of range");
-    if ((uint64_t)me.first_node + me.n_nodes > s->n_mesh_nodes) return fail(CRTB200_ERR_SCENE, "mesh node range out of bounds");
-    if ((uint64_t)me.first_leaf_ref + me.n_leaf_refs > s->n_mesh_leaf_refs) return fail(CRTB200_ERR_SCENE, "mesh leaf-ref range out of bounds");
+    if (trees && (uint64_t)me.first_node + me.n_nodes > s->n_mesh_nodes) return fail(CRTB200_ERR_SCENE, "mesh node range out of bounds");
+    if (trees && (uint64_t)me.first_leaf_ref + me.n_leaf_refs > s->n_mesh_leaf_refs) return fail(CRTB200_ERR_SCENE, "mesh leaf-ref range out of bounds");
     for (uint32_t t = 0; t < me.n_triangles; t++) tri_mesh[me.first_triangle + t] = m;
   }
   for (uint32_t t = 0; t < s->n_triangles; t++) {
@@ -718,10 +771,132 @@ static int upload_one(crtb200_ctx *c, const crtb200_scene *s) {
     const float *n = s->triangle_normal + 3 * (size_t)t;
     for (int k = 0; k < 3; k++) {
       const float *p = s->vertex_position + 3 * (size_t)iv[k];
-      geom[3 * (size_t)t + k] = make_float4(p[0], p[1], p[2], n[k]);
+      r.geom[3 * (size_t)t + k] = make_float4(p[0], p[1], p[2], n[k]);
     }
-    shade[t] = make_uint4(iv[0], iv[1], iv[2], tri_mesh[t]);
+    r.shade[t] = make_uint4(iv[0], iv[1], iv[2], tri_mesh[t]);
   }
+
+  r.vn.resize(s->n_vertices);
+  for (uint32_t v = 0; v < s->n_vertices; v++)
+    r.vn[v] = make_float4(s->vertex_normal[3 * (size_t)v], s->vertex_normal[3 * (size_t)v + 1], s->vertex_normal[3 * (size_t)v + 2], 0.f);
+  if (s->vertex_uv) {
+    r.uv.resize(s->n_vertices);
+    for (uint32_t v = 0; v < s->n_vertices; v++) r.uv[v] = make_float2(s->vertex_uv[3 * (size_t)v], s->vertex_uv[3 * (size_t)v + 1]);
+  }
+  r.mats.resize(s->n_materials);
+  for (uint32_t m = 0; m < s->n_materials; m++) {
+    const crtb200_material &mm = s->materials[m];
+    if (mm.texture != CRTB200_INVALID && mm.texture >= s->n_textures) return fail(CRTB200_ERR_SCENE, "material texture index out of range");
+    r.mats[m].type = mm.type;
+    r.mats[m].smooth = mm.smooth_shading;
+    r.mats[m].texture = mm.texture;
+    r.mats[m].ior = mm.ior;
+    for (int k = 0; k < 3; k++) r.mats[m].albedo[k] = mm.albedo[k];
+    r.mats[m].pad = 0.f;
+  }
+  r.texs.resize(s->n_textures);
+  for (uint32_t t = 0; t < s->n_textures; t++) {
+    const crtb200_texture &tt = s->textures[t];
+    DTexture &d = r.texs[t];
+    d.kind = tt.kind;
+    for (int k = 0; k < 3; k++) {
+      d.color_a[k] = tt.color_a[k];
+      d.color_b[k] = tt.color_b[k];
+    }
+    d.scalar = tt.scalar;
+    d.width = tt.width;
+    d.height = tt.height;
+    d.texel_offset = tt.texel_offset;
+    if (tt.kind == CRTB200_TEX_BITMAP) {
+      if (tt.width == 0 || tt.height == 0 || tt.texel_offset + (uint64_t)tt.width * tt.height > s->n_texels || !s->texels)
+        return fail(CRTB200_ERR_SCENE, "bitmap texture texel range out of bounds");
+    }
+  }
+  r.texels.assign(s->texels ? s->texels : nullptr, s->texels ? s->texels + 3 * s->n_texels : nullptr);
+  r.lights.resize(s->n_lights);
+  for (uint32_t l = 0; l < s->n_lights; l++) {
+    for (int k = 0; k < 3; k++) r.lights[l].pos[k] = s->lights[l].position[k];
+    r.lights[l].intensity = static_cast<float>(s->lights[l].intensity);  // RayTracer.cpp:320
+  }
+  return CRTB200_OK;
+}
+
+// The scene arena (nodes | leaf references | triangle geometry, one allocation, see crtb200_ctx::arena) for n_nodes
+// nodes, n_refs mesh leaf references and the scene's triangles.
+static int place_arena(crtb200_ctx *c, size_t n_nodes, size_t n_refs, size_t n_geom) {
+  auto al = [](size_t v) { return (v + 255) & ~(size_t)255; };
+  const size_t b_nodes = al(n_nodes * 2 * sizeof(float4)), b_refs = al(n_refs * sizeof(uint32_t)), b_geom = al(n_geom * sizeof(float4));
+  c->arena_used = b_nodes + b_refs + b_geom;
+  c->nodes_bytes = b_nodes;
+  CUDA_TRY(c->arena.ensure(std::max<size_t>(c->arena_used, 256)));
+  c->nodes_p = reinterpret_cast<float4 *>(c->arena.p);
+  c->leaf_refs_p = reinterpret_cast<uint32_t *>(c->arena.p + b_nodes);
+  c->tri_geom_p = reinterpret_cast<float4 *>(c->arena.p + b_nodes + b_refs);
+  return CRTB200_OK;
+}
+
+// Uploads the records, sets the device scene and the frame buffers; the trees (arena nodes and references, top_refs,
+// meshes, nested_ok) are in place.
+static int commit_scene(crtb200_ctx *c, const crtb200_scene *s, const SceneRecords &r, uint32_t n_nodes, uint32_t n_refs,
+                        uint32_t n_top_refs, uint32_t top_begin, uint32_t top_end) {
+  c->has_reflective = c->has_refractive = false;
+  for (uint32_t m = 0; m < s->n_meshes; m++) {
+    const uint32_t type = s->materials[s->meshes[m].material].type;
+    if (type == CRTB200_MAT_REFLECTIVE) c->has_reflective = true;
+    if (type == CRTB200_MAT_REFRACTIVE) c->has_refractive = true;
+  }
+  CUDA_TRY(c->tri_shade.upload(r.shade));
+  CUDA_TRY(c->vtx_normal.upload(r.vn));
+  if (!r.uv.empty()) CUDA_TRY(c->vtx_uv.upload(r.uv));
+  CUDA_TRY(c->materials.upload(r.mats));
+  CUDA_TRY(c->textures.upload(r.texs));
+  CUDA_TRY(c->texels.upload(r.texels));
+  CUDA_TRY(c->lights.upload(r.lights));
+  c->scene_bytes = (uint64_t)n_nodes * 32 + (uint64_t)n_refs * 4 + r.geom.size() * 16 + r.shade.size() * 16 + r.vn.size() * 16;
+  c->n_triangles = s->n_triangles;
+  c->n_nodes = n_nodes;
+  c->n_leaf_refs = n_refs;
+  c->n_top_refs = n_top_refs;
+
+  DScene &d = c->sc;
+  d.nodes = c->nodes_p;
+  d.leaf_refs = c->leaf_refs_p;
+  d.top_refs = c->top_refs.p;
+  d.tri_geom = c->tri_geom_p;
+  d.tri_shade = c->tri_shade.p;
+  d.vtx_normal = c->vtx_normal.p;
+  d.vtx_uv = r.uv.empty() ? nullptr : c->vtx_uv.p;
+  d.meshes = c->meshes.p;
+  d.materials = c->materials.p;
+  d.textures = c->textures.p;
+  d.texels = c->texels.p;
+  d.lights = c->lights.p;
+  d.n_lights = s->n_lights;
+  d.n_meshes = s->n_meshes;
+  d.top_begin = top_begin;
+  d.top_end = top_end;
+  d.width = s->width;
+  d.height = s->height;
+  for (int k = 0; k < 3; k++) d.bg[k] = s->background[k];
+  d.dedup_meshes = s->n_meshes <= 64 ? 1u : (s->n_meshes <= 512 ? 2u : 0u);
+  d.dedup_words = d.dedup_meshes == 2u ? (s->n_meshes + 31u) / 32u : 0u;
+
+  const size_t px = (size_t)s->width * s->height;
+  CUDA_TRY(c->frame.ensure(px * 3));
+  CUDA_TRY(cudaMemset(c->frame.p, 0, px * 3 * sizeof(float)));  // colorBuffer starts at (0,0,0), RayTracer.cpp:47-50
+  CUDA_TRY(c->frame8.ensure(px * 3));
+  CUDA_TRY(cudaMemset(c->frame8.p, 0, px * 3));
+  CUDA_TRY(c->stats_dev.ensure(48));
+  c->mask_valid = false;
+  c->cap_items = 0;
+  c->have_scene = true;
+  return CRTB200_OK;
+}
+
+static int upload_one(crtb200_ctx *c, const crtb200_scene *s) {
+  SceneRecords r;
+  int rc = pack_records(c, s, true, r);
+  if (rc) return rc;
   // trees: mesh trees first, top-level tree last, one node array
   std::vector<float4> nodes;
   bool nested_ok = true;
@@ -769,117 +944,322 @@ static int upload_one(crtb200_ctx *c, const crtb200_scene *s) {
   // culling margins (one pass over the leaf references and the triangles of each mesh; meshes in parallel would be easy,
   // but this is 0.1 s per million triangles)
   for (uint32_t m = 0; m < s->n_meshes; m++) meshes[m].cull_margin = mesh_cull_margin(s, s->meshes[m], nested_ok);
-
-  std::vector<float4> vn(s->n_vertices);
-  for (uint32_t v = 0; v < s->n_vertices; v++)
-    vn[v] = make_float4(s->vertex_normal[3 * (size_t)v], s->vertex_normal[3 * (size_t)v + 1], s->vertex_normal[3 * (size_t)v + 2], 0.f);
-  std::vector<float2> uv;
-  if (s->vertex_uv) {
-    uv.resize(s->n_vertices);
-    for (uint32_t v = 0; v < s->n_vertices; v++) uv[v] = make_float2(s->vertex_uv[3 * (size_t)v], s->vertex_uv[3 * (size_t)v + 1]);
-  }
-  std::vector<DMaterial> mats(s->n_materials);
-  c->has_reflective = c->has_refractive = false;
-  for (uint32_t m = 0; m < s->n_materials; m++) {
-    const crtb200_material &mm = s->materials[m];
-    if (mm.texture != CRTB200_INVALID && mm.texture >= s->n_textures) return fail(CRTB200_ERR_SCENE, "material texture index out of range");
-    mats[m].type = mm.type;
-    mats[m].smooth = mm.smooth_shading;
-    mats[m].texture = mm.texture;
-    mats[m].ior = mm.ior;
-    for (int k = 0; k < 3; k++) mats[m].albedo[k] = mm.albedo[k];
-    mats[m].pad = 0.f;
-  }
-  for (uint32_t m = 0; m < s->n_meshes; m++) {
-    const uint32_t type = s->materials[s->meshes[m].material].type;
-    if (type == CRTB200_MAT_REFLECTIVE) c->has_reflective = true;
-    if (type == CRTB200_MAT_REFRACTIVE) c->has_refractive = true;
-  }
-  std::vector<DTexture> texs(s->n_textures);
-  for (uint32_t t = 0; t < s->n_textures; t++) {
-    const crtb200_texture &tt = s->textures[t];
-    texs[t].kind = tt.kind;
-    for (int k = 0; k < 3; k++) {
-      texs[t].color_a[k] = tt.color_a[k];
-      texs[t].color_b[k] = tt.color_b[k];
-    }
-    texs[t].scalar = tt.scalar;
-    texs[t].width = tt.width;
-    texs[t].height = tt.height;
-    texs[t].texel_offset = tt.texel_offset;
-    if (tt.kind == CRTB200_TEX_BITMAP) {
-      if (tt.width == 0 || tt.height == 0 || tt.texel_offset + (uint64_t)tt.width * tt.height > s->n_texels || !s->texels)
-        return fail(CRTB200_ERR_SCENE, "bitmap texture texel range out of bounds");
-    }
-  }
-  std::vector<float> texels(s->texels ? s->texels : nullptr, s->texels ? s->texels + 3 * s->n_texels : nullptr);
-  std::vector<DLight> lights(s->n_lights);
-  for (uint32_t l = 0; l < s->n_lights; l++) {
-    for (int k = 0; k < 3; k++) lights[l].pos[k] = s->lights[l].position[k];
-    lights[l].intensity = static_cast<float>(s->lights[l].intensity);  // RayTracer.cpp:320
-  }
   std::vector<uint32_t> top_refs(s->top_leaf_refs, s->top_leaf_refs + s->n_top_leaf_refs);
 
-  {
-    auto al = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    const size_t b_nodes = al(nodes.size() * sizeof(float4)), b_refs = al(refs.size() * sizeof(uint32_t)),
-                 b_geom = al(geom.size() * sizeof(float4));
-    c->arena_used = b_nodes + b_refs + b_geom;
-    c->nodes_bytes = b_nodes;
-    CUDA_TRY(c->arena.ensure(std::max<size_t>(c->arena_used, 256)));
-    c->nodes_p = reinterpret_cast<float4 *>(c->arena.p);
-    c->leaf_refs_p = reinterpret_cast<uint32_t *>(c->arena.p + b_nodes);
-    c->tri_geom_p = reinterpret_cast<float4 *>(c->arena.p + b_nodes + b_refs);
-    if (!nodes.empty()) CUDA_TRY(cudaMemcpy(c->nodes_p, nodes.data(), nodes.size() * sizeof(float4), cudaMemcpyHostToDevice));
-    if (!refs.empty()) CUDA_TRY(cudaMemcpy(c->leaf_refs_p, refs.data(), refs.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    if (!geom.empty()) CUDA_TRY(cudaMemcpy(c->tri_geom_p, geom.data(), geom.size() * sizeof(float4), cudaMemcpyHostToDevice));
-  }
+  rc = place_arena(c, nodes.size() / 2, refs.size(), r.geom.size());
+  if (rc) return rc;
+  if (!nodes.empty()) CUDA_TRY(cudaMemcpy(c->nodes_p, nodes.data(), nodes.size() * sizeof(float4), cudaMemcpyHostToDevice));
+  if (!refs.empty()) CUDA_TRY(cudaMemcpy(c->leaf_refs_p, refs.data(), refs.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
+  if (!r.geom.empty()) CUDA_TRY(cudaMemcpy(c->tri_geom_p, r.geom.data(), r.geom.size() * sizeof(float4), cudaMemcpyHostToDevice));
   c->nested_ok = nested_ok;
   CUDA_TRY(c->top_refs.upload(top_refs));
-  CUDA_TRY(c->tri_shade.upload(shade));
-  CUDA_TRY(c->vtx_normal.upload(vn));
-  if (!uv.empty()) CUDA_TRY(c->vtx_uv.upload(uv));
   CUDA_TRY(c->meshes.upload(meshes));
-  CUDA_TRY(c->materials.upload(mats));
-  CUDA_TRY(c->textures.upload(texs));
-  CUDA_TRY(c->texels.upload(texels));
-  CUDA_TRY(c->lights.upload(lights));
-  c->scene_bytes = nodes.size() * 16 + refs.size() * 4 + geom.size() * 16 + shade.size() * 16 + vn.size() * 16;
-  c->n_triangles = s->n_triangles;
+  return commit_scene(c, s, r, (uint32_t)(nodes.size() / 2), (uint32_t)refs.size(), (uint32_t)top_refs.size(), top_begin, top_end);
+}
 
-  DScene &d = c->sc;
-  d.nodes = c->nodes_p;
-  d.leaf_refs = c->leaf_refs_p;
-  d.top_refs = c->top_refs.p;
-  d.tri_geom = c->tri_geom_p;
-  d.tri_shade = c->tri_shade.p;
-  d.vtx_normal = c->vtx_normal.p;
-  d.vtx_uv = uv.empty() ? nullptr : c->vtx_uv.p;
-  d.meshes = c->meshes.p;
-  d.materials = c->materials.p;
-  d.textures = c->textures.p;
-  d.texels = c->texels.p;
-  d.lights = c->lights.p;
-  d.n_lights = s->n_lights;
-  d.n_meshes = s->n_meshes;
-  d.top_begin = top_begin;
-  d.top_end = top_end;
-  d.width = s->width;
-  d.height = s->height;
-  for (int k = 0; k < 3; k++) d.bg[k] = s->background[k];
-  d.dedup_meshes = s->n_meshes <= 64 ? 1u : (s->n_meshes <= 512 ? 2u : 0u);
-  d.dedup_words = d.dedup_meshes == 2u ? (s->n_meshes + 31u) / 32u : 0u;
+// ---- device KD build: crtb200_upload_geometry (csrc/crt_build.cuh, DESIGN.md 3.11) -------------------------------
+// Scratch of one build, freed when the build returns (cudaFree synchronises the device); `peak` is what
+// crtb200_scene_trees reports.
+struct BuildScratch {
+  std::vector<std::pair<void *, size_t>> live_ptrs;
+  size_t live = 0, peak = 0;
+  template <typename T>
+  bool alloc(T *&p, size_t n) {
+    p = nullptr;
+    const size_t bytes = std::max<size_t>(n, 1) * sizeof(T);
+    if (cudaMalloc(reinterpret_cast<void **>(&p), bytes) != cudaSuccess) {
+      cudaGetLastError();  // an allocation failure is not sticky; clear it for the caller's later launches
+      p = nullptr;
+      return false;
+    }
+    live_ptrs.emplace_back(p, bytes);
+    live += bytes;
+    peak = std::max(peak, live);
+    return true;
+  }
+  void free(void *p) {
+    for (size_t i = 0; i < live_ptrs.size(); i++)
+      if (live_ptrs[i].first == p) {
+        cudaFree(p);
+        live -= live_ptrs[i].second;
+        live_ptrs.erase(live_ptrs.begin() + i);
+        return;
+      }
+  }
+  ~BuildScratch() {
+    for (auto &q : live_ptrs) cudaFree(q.first);
+  }
+};
 
-  const size_t px = (size_t)s->width * s->height;
-  CUDA_TRY(c->frame.ensure(px * 3));
-  CUDA_TRY(cudaMemset(c->frame.p, 0, px * 3 * sizeof(float)));  // colorBuffer starts at (0,0,0), RayTracer.cpp:47-50
-  CUDA_TRY(c->frame8.ensure(px * 3));
-  CUDA_TRY(cudaMemset(c->frame8.p, 0, px * 3));
-  CUDA_TRY(c->stats_dev.ensure(48));
-  c->mask_valid = false;
-  c->cap_items = 0;
-  c->have_scene = true;
-  return CRTB200_OK;
+// One level of the build: its nodes and, per node, child indices (into the next level), leaf reference count and
+// offset (into this level's leaf buffer), subtree node / reference counts, and the three numberings.
+struct BuildLevel {
+  uint32_t n = 0;
+  BNode *nodes = nullptr;
+  uint32_t *child = nullptr, *leaf_cnt = nullptr, *leaf_off = nullptr, *size = nullptr, *rsize = nullptr;
+  uint32_t *pre = nullptr, *vis = nullptr, *ref = nullptr, *leafbuf = nullptr;
+};
+
+struct BuildAdd2 {
+  __host__ __device__ uint2 operator()(const uint2 &a, const uint2 &b) const { return make_uint2(a.x + b.x, a.y + b.y); }
+};
+struct BuildAdd4 {
+  __host__ __device__ uint4 operator()(const uint4 &a, const uint4 &b) const {
+    return make_uint4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w);
+  }
+};
+
+static unsigned build_blocks(uint64_t n) { return (unsigned)std::max<uint64_t>(1, (n + 255) / 256); }
+
+// Builds the trees of `s` on c's GPU and uploads the scene; keep: also keep the reference-numbered trees for
+// crtb200_scene_trees.
+static int upload_geometry_one(crtb200_ctx *c, const crtb200_scene *s, bool keep) {
+  SceneRecords r;
+  int rc = pack_records(c, s, false, r);
+  if (rc) return rc;
+  const uint32_t M = s->n_meshes, T = M + 1;
+  std::vector<uint32_t> item_base(M + 1), mesh_tri(std::max(M, 1u), 0);
+  uint64_t items = 0;
+  for (uint32_t m = 0; m < M; m++) {
+    item_base[m] = (uint32_t)std::min<uint64_t>(items, 0xFFFFFFFFu);
+    mesh_tri[m] = s->meshes[m].first_triangle;
+    items += s->meshes[m].n_triangles;
+  }
+  if (items + M >= 0x7FFFFFFFull) return fail(CRTB200_ERR_SCENE, "scene too large for 31-bit indices");
+  item_base[M] = (uint32_t)items;
+  const uint32_t NI = (uint32_t)items, NE = NI + M;
+  cudaStream_t st = c->stream;
+
+  BuildScratch sc;
+  bool ok = true;
+  auto al = [&](auto *&p, size_t n) { ok = ok && sc.alloc(p, n); };
+  auto nomem = [&]() {
+    return fail(CRTB200_ERR_MEMORY, "device KD build: scratch does not fit on device " + std::to_string(c->device) + " (" +
+                                        std::to_string(sc.live) + " bytes allocated)");
+  };
+  float4 *geom;
+  uint32_t *d_item_base, *d_mesh_tri, *nested, *lelem, *lnode;
+  BBox *ebox;
+  unsigned long long *mslots, *slots;
+  al(geom, r.geom.size());
+  al(d_item_base, M + 1);
+  al(d_mesh_tri, mesh_tri.size());
+  al(ebox, NE);
+  al(mslots, 6 * (size_t)T);
+  al(slots, 4 * (size_t)T);
+  al(nested, 1);
+  al(lelem, NE);
+  al(lnode, NE);
+  std::vector<BuildLevel> lv(1);
+  auto alloc_level = [&](BuildLevel &L, uint32_t n) {
+    L.n = n;
+    uint32_t *w = nullptr;
+    al(L.nodes, n);
+    al(w, 9 * (size_t)n);
+    if (!ok) return;
+    L.child = w;
+    L.leaf_cnt = w + 2 * (size_t)n;
+    L.leaf_off = w + 3 * (size_t)n;
+    L.size = w + 4 * (size_t)n;
+    L.rsize = w + 5 * (size_t)n;
+    L.pre = w + 6 * (size_t)n;
+    L.vis = w + 7 * (size_t)n;
+    L.ref = w + 8 * (size_t)n;
+  };
+  alloc_level(lv[0], T);
+  if (!ok) return nomem();
+
+  cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+  CUDA_TRY(cudaEventCreate(&ev0));
+  if (cudaEventCreate(&ev1) != cudaSuccess) {
+    cudaEventDestroy(ev0);
+    return fail(CRTB200_ERR_CUDA, "cudaEventCreate failed");
+  }
+  struct Events {
+    cudaEvent_t a, b;
+    ~Events() {
+      cudaEventDestroy(a);
+      cudaEventDestroy(b);
+    }
+  } events{ev0, ev1};
+
+  if (!r.geom.empty()) CUDA_TRY(cudaMemcpyAsync(geom, r.geom.data(), r.geom.size() * sizeof(float4), cudaMemcpyHostToDevice, st));
+  CUDA_TRY(cudaMemcpyAsync(d_item_base, item_base.data(), item_base.size() * 4, cudaMemcpyHostToDevice, st));
+  CUDA_TRY(cudaMemcpyAsync(d_mesh_tri, mesh_tri.data(), mesh_tri.size() * 4, cudaMemcpyHostToDevice, st));
+  CUDA_TRY(cudaMemsetAsync(mslots, 0xFF, 6 * (size_t)T * sizeof(unsigned long long), st));
+  CUDA_TRY(cudaMemsetAsync(slots, 0, 4 * (size_t)T * sizeof(unsigned long long), st));
+  CUDA_TRY(cudaMemsetAsync(nested, 0xFF, sizeof(uint32_t), st));
+  CUDA_TRY(cudaEventRecord(ev0, st));
+
+  // boxes, roots and the level-0 listing
+  if (NI) k_build_item_boxes<<<build_blocks(NI), 256, 0, st>>>(geom, d_item_base, d_mesh_tri, M, NI, ebox, mslots);
+  if (M) k_build_roots<<<build_blocks(M), 256, 0, st>>>(d_item_base, M, NI, ebox, mslots, lv[0].nodes);
+  k_build_scene_box<<<1, 1, 0, st>>>(M, NI, ebox, lv[0].nodes);
+  if (NE) k_build_listing0<<<build_blocks(NE), 256, 0, st>>>(d_item_base, M, NI, lelem, lnode);
+  CUDA_TRY(cudaGetLastError());
+
+  // levels: classify, scan, count, scan, emit the children and scatter the listings
+  void *cub_tmp = nullptr;
+  size_t cub_bytes = 0;
+  auto cub_room = [&](size_t need) {
+    if (need <= cub_bytes) return;
+    if (cub_tmp) sc.free(cub_tmp);
+    cub_tmp = nullptr;
+    cub_bytes = 0;
+    uint8_t *p = nullptr;
+    al(p, need);
+    if (ok) {
+      cub_tmp = p;
+      cub_bytes = need;
+    }
+  };
+  uint32_t nL = NE;
+  for (uint32_t level = 0;; level++) {
+    const uint32_t nF = lv[level].n;
+    uint2 *S;
+    uint4 *NS;
+    al(S, (size_t)nL + 1);
+    al(NS, (size_t)nF + 1);
+    size_t b2 = 0, b4 = 0;
+    CUDA_TRY(cub::DeviceScan::ExclusiveScan(nullptr, b2, S, S, BuildAdd2(), make_uint2(0u, 0u), (int)nL + 1, st));
+    CUDA_TRY(cub::DeviceScan::ExclusiveScan(nullptr, b4, NS, NS, BuildAdd4(), make_uint4(0u, 0u, 0u, 0u), (int)nF + 1, st));
+    cub_room(std::max(b2, b4));
+    uint2 *flags;
+    uint4 *nc;
+    al(flags, (size_t)nL + 1);
+    al(nc, (size_t)nF + 1);
+    if (!ok) return nomem();
+    k_build_flags<<<build_blocks((uint64_t)nL + 1), 256, 0, st>>>(lv[level].nodes, lelem, lnode, nL, level, M, ebox, flags);
+    CUDA_TRY(cub::DeviceScan::ExclusiveScan(cub_tmp, b2, flags, S, BuildAdd2(), make_uint2(0u, 0u), (int)nL + 1, st));
+    k_build_counts<<<build_blocks((uint64_t)nF + 1), 256, 0, st>>>(lv[level].nodes, nF, level, M, S, nc);
+    CUDA_TRY(cub::DeviceScan::ExclusiveScan(cub_tmp, b4, nc, NS, BuildAdd4(), make_uint4(0u, 0u, 0u, 0u), (int)nF + 1, st));
+    uint4 tot;
+    CUDA_TRY(cudaMemcpyAsync(&tot, NS + nF, sizeof(uint4), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    sc.free(flags);
+    sc.free(nc);
+    if (tot.y >= 0x7FFFFFFFu) return fail(CRTB200_ERR_SCENE, "device KD build: a level lists more than 2^31 elements");
+    al(lv[level].leafbuf, tot.z);
+    uint32_t *next_elem = nullptr, *next_node = nullptr;
+    if (tot.x) {
+      lv.emplace_back();
+      alloc_level(lv.back(), tot.x);
+      al(next_elem, tot.y);
+      al(next_node, tot.y);
+    }
+    if (!ok) return nomem();
+    BuildLevel &L = lv[level];
+    BNode *next = tot.x ? lv[level + 1].nodes : nullptr;
+    k_build_emit<<<build_blocks(nF), 256, 0, st>>>(L.nodes, nF, level, M, S, NS, next, L.child, L.leaf_cnt, L.leaf_off);
+    if (nL) k_build_scatter<<<build_blocks(nL), 256, 0, st>>>(L.nodes, lelem, lnode, nL, level, M, S, NS, next_elem, next_node, L.leafbuf);
+    CUDA_TRY(cudaGetLastError());
+    sc.free(S);
+    sc.free(NS);
+    sc.free(lelem);
+    sc.free(lnode);
+    lelem = next_elem;
+    lnode = next_node;
+    nL = tot.y;
+    if (!tot.x) break;
+  }
+  const uint32_t D = (uint32_t)lv.size();
+
+  // numbering: subtree sizes bottom-up, then the per-tree bases on the host from the roots' sizes, then top-down
+  for (uint32_t l = D; l-- > 0;) {
+    const BuildLevel &L = lv[l];
+    const BuildLevel *N = l + 1 < D ? &lv[l + 1] : nullptr;
+    k_build_up<<<build_blocks(L.n), 256, 0, st>>>(L.nodes, L.n, M, L.child, L.leaf_cnt, L.size, L.rsize, N ? N->nodes : nullptr,
+                                                  N ? N->size : nullptr, N ? N->rsize : nullptr, nested);
+  }
+  CUDA_TRY(cudaGetLastError());
+  std::vector<uint32_t> root_size(T), root_rsize(T);
+  CUDA_TRY(cudaMemcpyAsync(root_size.data(), lv[0].size, T * 4, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaMemcpyAsync(root_rsize.data(), lv[0].rsize, T * 4, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaStreamSynchronize(st));
+  std::vector<uint32_t> node_base(T), ref_base(T);
+  uint64_t n_nodes = 0, n_refs = 0;
+  for (uint32_t t = 0; t < T; t++) {
+    node_base[t] = (uint32_t)std::min<uint64_t>(n_nodes, 0xFFFFFFFFu);
+    n_nodes += root_size[t];
+    ref_base[t] = t < M ? (uint32_t)std::min<uint64_t>(n_refs, 0xFFFFFFFFu) : 0u;
+    if (t < M) n_refs += root_rsize[t];
+  }
+  if (n_nodes >= 0x7FFFFFF0u || n_refs >= 0x7FFFFFF0u) return fail(CRTB200_ERR_SCENE, "scene too large for 31-bit indices");
+  const uint32_t n_top_refs = root_rsize[M], top_begin = node_base[M];
+  uint32_t *d_node_base, *d_ref_base;
+  al(d_node_base, T);
+  al(d_ref_base, T);
+  if (!ok) return nomem();
+  CUDA_TRY(cudaMemcpyAsync(d_node_base, node_base.data(), T * 4, cudaMemcpyHostToDevice, st));
+  CUDA_TRY(cudaMemcpyAsync(d_ref_base, ref_base.data(), T * 4, cudaMemcpyHostToDevice, st));
+  CUDA_TRY(cudaMemsetAsync(lv[0].pre, 0, 3 * (size_t)T * sizeof(uint32_t), st));  // pre, vis, ref of the roots
+  for (uint32_t l = 0; l + 1 < D; l++) {
+    const BuildLevel &L = lv[l], &N = lv[l + 1];
+    k_build_down<<<build_blocks(L.n), 256, 0, st>>>(L.n, L.child, L.pre, L.vis, L.ref, N.size, N.rsize, N.pre, N.vis, N.ref);
+  }
+  CUDA_TRY(cudaGetLastError());
+
+  // the scene's device arrays: arena, top-level references, meshes (the margins follow), kept trees
+  CUDA_TRY(cudaStreamSynchronize(st));
+  rc = place_arena(c, n_nodes, n_refs, r.geom.size());
+  if (rc) return rc;
+  if (!r.geom.empty()) CUDA_TRY(cudaMemcpyAsync(c->tri_geom_p, geom, r.geom.size() * sizeof(float4), cudaMemcpyDeviceToDevice, st));
+  CUDA_TRY(c->top_refs.ensure(std::max<uint32_t>(n_top_refs, 1)));
+  std::vector<DMesh> meshes(M);
+  for (uint32_t m = 0; m < M; m++) {
+    meshes[m].node_begin = node_base[m];
+    meshes[m].node_end = node_base[m] + root_size[m];
+    meshes[m].material = s->meshes[m].material;
+    meshes[m].first_triangle = s->meshes[m].first_triangle;
+    meshes[m].cull_margin = std::numeric_limits<float>::infinity();
+  }
+  CUDA_TRY(c->meshes.upload(meshes));
+  if (keep) {
+    if (c->kd_nodes.ensure(std::max<uint64_t>(n_nodes, 1)) != cudaSuccess || c->kd_refs.ensure(std::max<uint64_t>(n_refs, 1)) != cudaSuccess) {
+      cudaGetLastError();
+      return fail(CRTB200_ERR_MEMORY, "device KD build: the built trees do not fit on device " + std::to_string(c->device));
+    }
+  }
+  for (uint32_t l = 0; l < D; l++) {
+    const BuildLevel &L = lv[l];
+    const BuildLevel *N = l + 1 < D ? &lv[l + 1] : nullptr;
+    k_build_write<<<build_blocks(L.n), 256, 0, st>>>(L.nodes, L.n, M, NI, L.child, L.leaf_cnt, L.leaf_off, L.leafbuf, L.size, L.pre, L.vis,
+                                                     L.ref, N ? N->pre : nullptr, N ? N->vis : nullptr, d_node_base, d_ref_base,
+                                                     d_item_base, d_mesh_tri, geom, c->nodes_p, c->leaf_refs_p, c->top_refs.p,
+                                                     keep ? c->kd_nodes.p : nullptr, keep ? c->kd_refs.p : nullptr, slots);
+  }
+  if (NI) k_build_tri_margin<<<build_blocks(NI), 256, 0, st>>>(geom, d_item_base, d_mesh_tri, M, NI, slots);
+  if (M) k_build_margins<<<build_blocks(M), 256, 0, st>>>(M, slots, nested, c->meshes.p);
+  CUDA_TRY(cudaGetLastError());
+  CUDA_TRY(cudaEventRecord(ev1, st));
+  uint32_t nested_h = 0;
+  CUDA_TRY(cudaMemcpyAsync(&nested_h, nested, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaStreamSynchronize(st));
+  float build_ms = 0.f;
+  cudaEventElapsedTime(&build_ms, ev0, ev1);
+  c->nested_ok = nested_h != 0;  // every tree is at most 26 levels deep: k_coop's limit of 40 always holds
+
+  if (keep) {
+    c->kd_meshes.assign(s->meshes, s->meshes + M);
+    for (uint32_t m = 0; m < M; m++) {
+      c->kd_meshes[m].first_node = node_base[m];
+      c->kd_meshes[m].n_nodes = root_size[m];
+      c->kd_meshes[m].first_leaf_ref = ref_base[m];
+      c->kd_meshes[m].n_leaf_refs = root_rsize[m];
+    }
+    crtb200_trees &k = c->kd_counts;
+    k = crtb200_trees{};
+    k.n_meshes = M;
+    k.n_mesh_nodes = top_begin;
+    k.n_mesh_leaf_refs = (uint32_t)n_refs;
+    k.n_top_nodes = root_size[M];
+    k.n_top_leaf_refs = n_top_refs;
+    k.peak_scratch_bytes = sc.peak;
+    k.build_ms = build_ms;
+  }
+  rc = commit_scene(c, s, r, (uint32_t)n_nodes, (uint32_t)n_refs, n_top_refs, top_begin, (uint32_t)n_nodes);
+  if (rc == CRTB200_OK && keep) c->trees_built = true;
+  return rc;
 }
 
 // ---- frame planning ------------------------------------------------------------------------------------------
@@ -2182,6 +2562,64 @@ int crtb200_generate_rays(crtb200_ctx *c, const crtb200_camera *cam, float *rays
   cudaError_t e = cudaMemcpyAsync(rays_out, d.p, n * 6 * sizeof(float), cudaMemcpyDeviceToHost, c->stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
   d.release();
+  CUDA_TRY(e);
+  return CRTB200_OK;
+}
+
+int crtb200_scene_trees(crtb200_ctx *c, crtb200_trees *t) {
+  ErrScope scope(c);
+  if (!c || !t) return fail(CRTB200_ERR_ARG, "null argument");
+  if (!c->trees_built) return fail(CRTB200_ERR_STATE, "the context's scene was not uploaded with crtb200_upload_geometry");
+  CUDA_TRY(cudaSetDevice(c->device));
+  const crtb200_trees &k = c->kd_counts;
+  t->n_meshes = k.n_meshes;
+  t->n_mesh_nodes = k.n_mesh_nodes;
+  t->n_mesh_leaf_refs = k.n_mesh_leaf_refs;
+  t->n_top_nodes = k.n_top_nodes;
+  t->n_top_leaf_refs = k.n_top_leaf_refs;
+  t->reserved = 0;
+  t->peak_scratch_bytes = k.peak_scratch_bytes;
+  t->build_ms = k.build_ms;
+  if (t->meshes && k.n_meshes) std::memcpy(t->meshes, c->kd_meshes.data(), k.n_meshes * sizeof(crtb200_mesh));
+  cudaError_t e = cudaSuccess;
+  auto get = [&](void *dst, const void *src, size_t bytes) {
+    if (dst && bytes && e == cudaSuccess) e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, c->stream);
+  };
+  get(t->mesh_nodes, c->kd_nodes.p, (size_t)k.n_mesh_nodes * sizeof(crtb200_kdnode));
+  get(t->mesh_leaf_refs, c->kd_refs.p, (size_t)k.n_mesh_leaf_refs * 4);
+  get(t->top_nodes, c->kd_nodes.p + k.n_mesh_nodes, (size_t)k.n_top_nodes * sizeof(crtb200_kdnode));
+  get(t->top_leaf_refs, c->top_refs.p, (size_t)k.n_top_leaf_refs * 4);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+  CUDA_TRY(e);
+  return CRTB200_OK;
+}
+
+int crtb200_debug_scene_layout(crtb200_ctx *c, int device_index, crtb200_scene_layout *l) {
+  ErrScope scope(c);
+  if (!c || !l) return fail(CRTB200_ERR_ARG, "null argument");
+  if (device_index < 0 || (size_t)device_index > c->peers.size()) return fail(CRTB200_ERR_ARG, "device_index out of range");
+  crtb200_ctx *x = device_index ? c->peers[device_index - 1] : c;
+  if (!x->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
+  static_assert(sizeof(DMesh) == 20, "crtb200_scene_layout.meshes holds 5 words per mesh");
+  l->n_nodes = x->n_nodes;
+  l->n_leaf_refs = x->n_leaf_refs;
+  l->n_top_refs = x->n_top_refs;
+  l->n_meshes = x->sc.n_meshes;
+  l->top_begin = x->sc.top_begin;
+  l->top_end = x->sc.top_end;
+  l->nested_ok = x->nested_ok ? 1u : 0u;
+  l->reserved = 0;
+  CUDA_TRY(cudaSetDevice(x->device));
+  cudaError_t e = cudaSuccess;
+  auto get = [&](void *dst, const void *src, size_t bytes) {
+    if (dst && bytes && e == cudaSuccess) e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, x->stream);
+  };
+  get(l->nodes, x->nodes_p, (size_t)x->n_nodes * 32);
+  get(l->leaf_refs, x->leaf_refs_p, (size_t)x->n_leaf_refs * 4);
+  get(l->top_refs, x->top_refs.p, (size_t)x->n_top_refs * 4);
+  get(l->meshes, x->meshes.p, (size_t)x->sc.n_meshes * sizeof(DMesh));
+  if (e == cudaSuccess) e = cudaStreamSynchronize(x->stream);
+  cudaSetDevice(c->device);
   CUDA_TRY(e);
   return CRTB200_OK;
 }

@@ -11,8 +11,8 @@ using namespace crt;
 
 struct crtfe_scene {
   Scene scene;
-  FlatScene flat;
-  bool flattened = false;
+  FlatScene flat, geometry;  // crtfe_scene_flatten / crtfe_scene_flatten_geometry, each built once
+  bool flattened = false, geometry_flattened = false;
 };
 struct crtfe_tracer {
   std::unique_ptr<RayTracer> tracer;
@@ -123,6 +123,17 @@ int crtfe_scene_flatten(crtfe_scene *s, uint32_t threads, const crtb200_scene **
     }
     *out = &s->flat.abi;
     if (seconds) *seconds = s->flat.buildSeconds;
+  })
+}
+int crtfe_scene_flatten_geometry(crtfe_scene *s, const crtb200_scene **out, double *seconds) {
+  if (!s || !out) return fail("null argument");
+  CRTFE_TRY({
+    if (!s->geometry_flattened) {
+      buildFlatScene(s->scene, s->geometry, 1, false);
+      s->geometry_flattened = true;
+    }
+    *out = &s->geometry.abi;
+    if (seconds) *seconds = s->geometry.buildSeconds;
   })
 }
 int crtfe_rectangles(uint32_t w, uint32_t h, uint32_t mode, uint32_t bucket, uint32_t hw, crtb200_rect *out,

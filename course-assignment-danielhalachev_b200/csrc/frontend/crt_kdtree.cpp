@@ -156,7 +156,7 @@ static inline void grow(Box &b, const Vector &p) {  // std::min / std::max as wr
   }
 }
 
-void buildFlatScene(const Scene &scene, FlatScene &out, unsigned threads) {
+void buildFlatScene(const Scene &scene, FlatScene &out, unsigned threads, bool trees) {
   auto t0 = std::chrono::steady_clock::now();
   if (threads == 0) threads = std::max(1u, std::thread::hardware_concurrency());
   out = FlatScene();
@@ -187,20 +187,28 @@ void buildFlatScene(const Scene &scene, FlatScene &out, unsigned threads) {
     }
     // per-triangle boxes (BoundingBox(const Triangle&), BoundingBox.h:50-58) and the mesh root box
     // (BoundingBox(const std::vector<Triangle>&), BoundingBox.h:26-34: only vertices referenced by triangles)
-    std::vector<Box> triBoxes(fm.n_triangles);
+    std::vector<Box> triBoxes(trees ? fm.n_triangles : 0);
     Box root = emptyBox();
     for (uint32_t t = 0; t < fm.n_triangles; t++) {
       Box b = emptyBox();
       for (int k = 0; k < 3; k++) {
         const uint32_t vi = mesh.indices[3 * t + k];
-        grow(b, mesh.positions[vi]);
-        grow(root, mesh.positions[vi]);
-        grow(sceneBox, mesh.positions[vi]);
+        if (trees) {
+          grow(b, mesh.positions[vi]);
+          grow(root, mesh.positions[vi]);
+          grow(sceneBox, mesh.positions[vi]);
+        }
         out.triangleVertex.push_back(vtxBase + vi);
       }
-      triBoxes[t] = b;
+      if (trees) triBoxes[t] = b;
       const Vector &fn = mesh.faceNormals[t];
       out.triangleNormal.insert(out.triangleNormal.end(), {fn.x, fn.y, fn.z});
+    }
+    vtxBase += fm.n_vertices;
+    triBase += fm.n_triangles;
+    if (!trees) {  // geometry only (crtb200_upload_geometry builds the trees): tree fields 0
+      fm.first_node = fm.n_nodes = fm.first_leaf_ref = fm.n_leaf_refs = 0;
+      continue;
     }
     // TriangleKDTree(mesh, 25, 8)  AccelerationStructure.h:10-11
     KDTreeData tree = buildKDTree(triBoxes, root, 25, 8, threads);
@@ -212,13 +220,13 @@ void buildFlatScene(const Scene &scene, FlatScene &out, unsigned threads) {
     out.meshLeafRefs.insert(out.meshLeafRefs.end(), tree.refs.begin(), tree.refs.end());
     // ObjectKDTreeSubTree::getBoundingBox = tree root box  AccelerationStructure.cpp:21-23
     meshBoxes[mi] = root;
-    vtxBase += fm.n_vertices;
-    triBase += fm.n_triangles;
   }
-  // ObjectKDTree(scene, 25, 4): root box = BoundingBox(scene)  AccelerationStructure.cpp:27-45, BoundingBox.h:36-48
-  KDTreeData top = buildKDTree(meshBoxes, sceneBox, 25, 4, 1);
-  out.topNodes = std::move(top.nodes);
-  out.topLeafRefs = std::move(top.refs);
+  if (trees) {
+    // ObjectKDTree(scene, 25, 4): root box = BoundingBox(scene)  AccelerationStructure.cpp:27-45, BoundingBox.h:36-48
+    KDTreeData top = buildKDTree(meshBoxes, sceneBox, 25, 4, 1);
+    out.topNodes = std::move(top.nodes);
+    out.topLeafRefs = std::move(top.refs);
+  }
 
   for (const Material &m : scene.materials) {
     crtb200_material fm;
@@ -277,13 +285,13 @@ void buildFlatScene(const Scene &scene, FlatScene &out, unsigned threads) {
   a.n_lights = static_cast<uint32_t>(out.lights.size());
   a.lights = out.lights.data();
   a.n_mesh_nodes = static_cast<uint32_t>(out.meshNodes.size());
-  a.mesh_nodes = out.meshNodes.data();
+  a.mesh_nodes = trees ? out.meshNodes.data() : nullptr;
   a.n_mesh_leaf_refs = static_cast<uint32_t>(out.meshLeafRefs.size());
-  a.mesh_leaf_refs = out.meshLeafRefs.data();
+  a.mesh_leaf_refs = trees ? out.meshLeafRefs.data() : nullptr;
   a.n_top_nodes = static_cast<uint32_t>(out.topNodes.size());
-  a.top_nodes = out.topNodes.data();
+  a.top_nodes = trees ? out.topNodes.data() : nullptr;
   a.n_top_leaf_refs = static_cast<uint32_t>(out.topLeafRefs.size());
-  a.top_leaf_refs = out.topLeafRefs.data();
+  a.top_leaf_refs = trees ? out.topLeafRefs.data() : nullptr;
   out.buildSeconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
 }
 

@@ -45,7 +45,8 @@ struct FlatScene {
   double buildSeconds = 0;
 };
 
-// AccelerationStructure(scene) + flattening.  threads = 0 -> hardware_concurrency.
-void buildFlatScene(const Scene &scene, FlatScene &out, unsigned threads = 0);
+// AccelerationStructure(scene) + flattening.  threads = 0 -> hardware_concurrency.  trees = false: the flattened arrays
+// alone (tree counts 0, tree arrays NULL, the meshes' tree fields 0), for crtb200_upload_geometry.
+void buildFlatScene(const Scene &scene, FlatScene &out, unsigned threads = 0, bool trees = true);
 
 }  // namespace crt

@@ -52,7 +52,7 @@ def build_core(force: bool = False, verbose: bool = False, extra: list[str] | No
         src = os.path.join(CSRC, "crtb200_core.cu")
         _run([nvcc_path(), *NVCC_FLAGS, *(extra or []), "-o", out, src], verbose)
         return out
-    srcs = [os.path.join(CSRC, f) for f in ("crtb200_core.cu", "crt_kernels.cuh", "crt_device.cuh", "crt_powf5.h", "crt_sampling.h")]
+    srcs = [os.path.join(CSRC, f) for f in ("crtb200_core.cu", "crt_kernels.cuh", "crt_device.cuh", "crt_powf5.h", "crt_sampling.h", "crt_build.cuh")]
     srcs.append(os.path.join(ROOT, "include", "crtb200.h"))
     if force or not _newer(CORE_SO, srcs):
         _run([nvcc_path(), *NVCC_FLAGS, *(extra or []), "-o", CORE_SO, srcs[0]], verbose)

@@ -260,8 +260,8 @@ int crtb200_last_sampling_stats(crtb200_ctx *ctx, crtb200_sampling_stats *stats)
  * per-pixel accumulator of 40 bytes per pixel on each GPU (that GPU's tile shard).  After steps totalling n samples,
  * crtb200_accum_read returns bit for bit what crtb200_render returns with the same camera and options and
  * rays_per_pixel = n, and the steps' ray counts (and, with count_work = 1, test counts) add up to that frame's.
- * Ordinary renders and crtb200_set_sampling between steps do not affect the session; crtb200_upload_scene and
- * crtb200_destroy end it.  Every call but begin fails with CRTB200_ERR_STATE without a session. */
+ * Ordinary renders and crtb200_set_sampling between steps do not affect the session; crtb200_upload_scene,
+ * crtb200_upload_geometry and crtb200_destroy end it.  Every call but begin fails with CRTB200_ERR_STATE without a session. */
 
 /* replaces: the per-pixel sample loop's set-up, RayTracer.cpp:90-104 (no counterpart: see above).  Snapshots camera,
  * options (the rects array is copied) and sampling (rays_per_pixel is ignored) and starts at 0 samples; a session in
@@ -332,6 +332,48 @@ int crtb200_accum_load_counts(crtb200_ctx *ctx, const float *sum, const float *s
 /* replaces: the data RayTracer keeps in `scene`, `boundingBox`, `accelerationStructure` (RayTracer.h:64-67).
  * Copies + re-lays-out everything to device SoA during the call (host flattener H1). */
 int crtb200_upload_scene(crtb200_ctx *ctx, const crtb200_scene *scene);
+
+/* replaces: TriangleKDTree(mesh, 25, 8) per mesh and ObjectKDTree(scene, 25, 4) (AccelerationStructure.h:10-11,
+ * AccelerationStructure.cpp:12-50) plus crtb200_upload_scene: the KD trees are built on the device (DESIGN.md 3.11), one
+ * replica per GPU of the context, node for node the trees of the host front end (csrc/frontend/crt_kdtree.cpp), and the
+ * context is left exactly as crtb200_upload_scene leaves it given those trees.  The scene's n_mesh_nodes,
+ * n_mesh_leaf_refs, n_top_nodes and n_top_leaf_refs must be 0 and their pointers NULL (else CRTB200_ERR_ARG); the tree
+ * fields of crtb200_mesh are ignored; every other array is validated as by crtb200_upload_scene, with the same codes.
+ * Ends a progressive session.  CRTB200_ERR_MEMORY when the build's scratch does not fit; it is freed before returning. */
+int crtb200_upload_geometry(crtb200_ctx *ctx, const crtb200_scene *scene);
+
+/* The trees of the last crtb200_upload_geometry, in the reference's numbering and the crtb200_scene layout. */
+typedef struct crtb200_trees {
+  uint32_t n_meshes, n_mesh_nodes, n_mesh_leaf_refs, n_top_nodes, n_top_leaf_refs;
+  uint32_t reserved;
+  uint64_t peak_scratch_bytes; /* the build's device scratch at its peak, on the first GPU of the context             */
+  double build_ms;             /* CUDA-event time of the build on that GPU, from its first to its last kernel          */
+  crtb200_mesh *meshes;        /* n_meshes records as uploaded, with first_node, n_nodes, first_leaf_ref, n_leaf_refs */
+  crtb200_kdnode *mesh_nodes;  /* n_mesh_nodes                                                                      */
+  uint32_t *mesh_leaf_refs;    /* n_mesh_leaf_refs mesh-local triangle indices                                      */
+  crtb200_kdnode *top_nodes;   /* n_top_nodes                                                                       */
+  uint32_t *top_leaf_refs;     /* n_top_leaf_refs mesh indices                                                      */
+} crtb200_trees;
+/* replaces: the AccelerationStructure a RayTracer holds (RayTracer.h:65), read back.  Fills the counts, then every
+ * non-NULL array (sized from a call with NULL arrays).  CRTB200_ERR_STATE unless the context's scene came from
+ * crtb200_upload_geometry. */
+int crtb200_scene_trees(crtb200_ctx *ctx, crtb200_trees *trees);
+
+/* The device scene state of one GPU of the context, as the traversal kernels read it (csrc/crt_device.cuh). */
+typedef struct crtb200_scene_layout {
+  uint32_t n_nodes, n_leaf_refs, n_top_refs, n_meshes;
+  uint32_t top_begin, top_end; /* the top-level tree's node range                                              */
+  uint32_t nested_ok;          /* 1 = culling and the tail hand-off are enabled for the scene (DESIGN.md 3.7) */
+  uint32_t reserved;
+  uint32_t *nodes;     /* 8 words per 32-byte node of the visiting-order array: min.xyz, a, max.xyz, b   */
+  uint32_t *leaf_refs; /* global triangle ids                                                           */
+  uint32_t *top_refs;  /* mesh ids                                                                      */
+  uint32_t *meshes;    /* 5 words per mesh: node_begin, node_end, material, first_triangle, cull_margin bits */
+} crtb200_scene_layout;
+/* Test hook: copies GPU device_index's (0 = the first of the context) scene state to the host -- counts always, then
+ * every non-NULL array -- so tests can compare crtb200_upload_geometry with crtb200_upload_scene bit for bit.
+ * CRTB200_ERR_STATE without a scene. */
+int crtb200_debug_scene_layout(crtb200_ctx *ctx, int device_index, crtb200_scene_layout *layout);
 
 /* replaces: RayTracer::render's scheduler switch + renderRectangle pixel loop (RayTracer.cpp:82-112,209-286).
  * rgb_out: H*W*3 float32 row-major, host memory, = the colorBuffer render() returns (RayTracer.cpp:297).  Pixels not

@@ -3,6 +3,7 @@
  * (csrc/frontend/crt_scene.hpp, crt_raytracer.hpp); these wrappers expose exactly that API:
  *   SceneParser::parseScene (SceneParser.cpp:39-66)      -> crtfe_scene_load
  *   AccelerationStructure(scene) (AccelerationStructure.cpp:27-50) + flattening -> crtfe_scene_flatten
+ *   flattening without the trees (built on the GPU by crtb200_upload_geometry) -> crtfe_scene_flatten_geometry
  *   RayTracer(scene) / setCamera / render / exportPPM (RayTracer.h:97-101) -> crtfe_tracer_*
  *   Camera::pan/tilt/roll/truck (Camera.cpp:33-70)       -> crtfe_camera_*
  * All functions return 0 on success, negative on error; crtfe_last_error() gives the message. */
@@ -33,6 +34,9 @@ int crtfe_scene_free(crtfe_scene *scene);
 int crtfe_scene_get_info(const crtfe_scene *scene, crtfe_scene_info *info);
 /* builds the KD trees and the flattened arrays (idempotent); *out stays valid until crtfe_scene_free */
 int crtfe_scene_flatten(crtfe_scene *scene, uint32_t threads, const crtb200_scene **out, double *build_seconds);
+/* the same flattened arrays without the KD build, for crtb200_upload_geometry: tree counts 0, tree arrays NULL, the
+ * meshes' tree fields 0 (idempotent; independent of crtfe_scene_flatten's result, which it leaves as it is) */
+int crtfe_scene_flatten_geometry(crtfe_scene *scene, const crtb200_scene **out, double *seconds);
 
 /* rectangle grid of the reference's schedulers (RayTracer.cpp:114-158); mode = RenderOptimization value (10 = B200) */
 int crtfe_rectangles(uint32_t width, uint32_t height, uint32_t mode, uint32_t bucket_size, uint32_t hw_threads,
