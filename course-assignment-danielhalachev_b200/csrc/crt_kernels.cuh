@@ -1464,19 +1464,28 @@ struct HitRec {
   int mesh, tri;
   float t;
 };
+// A global triangle in public numbering: h.mesh and h.tri (the triangle within its mesh), -1 and -1 for CRT_INVALID.
+// h.t is the caller's.
+CRT_DI void public_tri(const DScene &sc, uint32_t tri, HitRec &h) {
+  h.mesh = h.tri = -1;
+  if (tri != CRT_INVALID) {
+    const uint32_t m = sc.tri_shade[tri].w;
+    h.mesh = (int)m;
+    h.tri = (int)(tri - sc.meshes[m].first_triangle);
+  }
+}
+// The frame stores of k_store and k_accum_read.  colour(i) is level-0 item i's colour, hit(i) its HitRec; both are only
+// called for items that are pixels of the frame (and hit only when `hits` is not null).
 // A warp holds one 8x4 tile (items are tile-major and chunks start on tile boundaries).  When the whole tile is inside
 // the frame its four 96-byte rows leave as 16-byte stores (24 lanes x float4; PPMColor: 12 lanes x 8 bytes), staged
 // through shared memory: a third of the store instructions, and -- what matters when `rgb` is the frame of another GPU
 // (crtb200_create_multi, shard_full_frame) -- NVLink packets of 16 bytes instead of 4.  Partial tiles, odd widths and
 // unaligned frames take the scalar path.
-__global__ void __launch_bounds__(256) k_store(const DScene sc, const Frame fr, const Levels lv, float *__restrict__ rgb,
-                                              uint8_t *__restrict__ rgb8, HitRec *__restrict__ hits,
-                                              float *__restrict__ slab) {
+template <class Colour, class Hit>
+CRT_DI void store_items(const DScene &sc, const Frame &fr, float *__restrict__ rgb, uint8_t *__restrict__ rgb8,
+                        HitRec *__restrict__ hits, float *__restrict__ slab, const Colour &colour, const Hit &hit) {
   __shared__ __align__(16) float s_f[8][96];
   __shared__ __align__(8) uint8_t s_b[8][96];
-  // shadow rays traced for this chunk = diffuse hits x lights (one per pair even when cos = 0, RayTracer.cpp:314-317)
-  if (blockIdx.x == 0 && threadIdx.x == 0)
-    atomicAdd(&lv.stats[1], (unsigned long long)lv.counts[CRT_MAX_LEVELS] * sc.n_lights);
   const uint32_t lane = lane_id(), w = threadIdx.x >> 5;
   const bool aligned = (sc.width & 7u) == 0u && (fr.item_begin & 31u) == 0u && (reinterpret_cast<uintptr_t>(rgb) & 15u) == 0u &&
                        (reinterpret_cast<uintptr_t>(rgb8) & 7u) == 0u && (reinterpret_cast<uintptr_t>(slab) & 15u) == 0u;
@@ -1484,7 +1493,7 @@ __global__ void __launch_bounds__(256) k_store(const DScene sc, const Frame fr, 
     const uint32_t i = base + lane;
     uint32_t row = 0, col = 0;
     const bool valid = i < fr.n_items0 && item_pixel(fr, sc, fr.item_begin + i, row, col);
-    const float4 c = valid ? lv.color[lv.offset[0] + i] : make_float4(0.f, 0.f, 0.f, 0.f);
+    const float4 c = valid ? colour(i) : make_float4(0.f, 0.f, 0.f, 0.f);
     const bool whole = aligned && base + 32u <= fr.n_items0;                 // all 32 items exist (slab path)
     const bool full = whole && __all_sync(CRT_FULL_MASK, valid);             // ... and are pixels of the frame
     const size_t pix = (size_t)row * sc.width + col;
@@ -1532,65 +1541,96 @@ __global__ void __launch_bounds__(256) k_store(const DScene sc, const Frame fr, 
       rgb8[3 * pix + 1] = quantize(c.y);
       rgb8[3 * pix + 2] = quantize(c.z);
     }
-    if (hits) {
-      const uint32_t tri = lv.hit_tri[lv.offset[0] + i];
-      HitRec h;
-      if (tri == CRT_INVALID) {
-        h.mesh = -1;
-        h.tri = -1;
-        h.t = 0.0f;
-      } else {
-        const uint32_t m = sc.tri_shade[tri].w;
-        h.mesh = (int)m;
-        h.tri = (int)(tri - sc.meshes[m].first_triangle);
-        h.t = lv.hit_t[lv.offset[0] + i];
-      }
-      hits[pix] = h;
-    }
+    if (hits) hits[pix] = hit(i);
   }
 }
 
+__global__ void __launch_bounds__(256) k_store(const DScene sc, const Frame fr, const Levels lv, float *__restrict__ rgb,
+                                              uint8_t *__restrict__ rgb8, HitRec *__restrict__ hits,
+                                              float *__restrict__ slab) {
+  // shadow rays traced for this chunk = diffuse hits x lights (one per pair even when cos = 0, RayTracer.cpp:314-317)
+  if (blockIdx.x == 0 && threadIdx.x == 0)
+    atomicAdd(&lv.stats[1], (unsigned long long)lv.counts[CRT_MAX_LEVELS] * sc.n_lights);
+  store_items(
+      sc, fr, rgb, rgb8, hits, slab, [&](uint32_t i) { return lv.color[lv.offset[0] + i]; },
+      [&](uint32_t i) {
+        const uint32_t tri = lv.hit_tri[lv.offset[0] + i];
+        HitRec h;
+        public_tri(sc, tri, h);
+        h.t = tri == CRT_INVALID ? 0.0f : lv.hit_t[lv.offset[0] + i];
+        return h;
+      });
+}
+
 // ------------------------------------------------------------------------------------------------------------
-// Progressive sessions (crtb200_accum_*, DESIGN.md 3.10.1).  The session's accumulator holds, per shard item (item_begin
-// + i, so that chunks never collide), S = ((0 + c_0) + c_1) + ..., Q = ((0 + c_0 c_0) + c_1 c_1) + ... and sample 0's
-// primary hit {global triangle, bits(t)}.  S and Q start at +0, so S is k_sample_acc's running sum bit for bit.
+// Progressive sessions (crtb200_accum_*, DESIGN.md 3.10.1 / 3.10.2).  The session's accumulator holds, per shard item
+// (item_begin + i, so that chunks never collide), S = ((0 + c_0) + c_1) + ..., Q = ((0 + c_0 c_0) + c_1 c_1) + ... and
+// sample 0's primary hit {global triangle, bits(t)}.  S and Q start at +0, so S is k_sample_acc's running sum bit for
+// bit.  The unused w lanes hold the pixel's sample count n_p (S.w, as uint32 bits) and, in adaptive sessions, its active
+// flag (Q.w: 1 = still sampling, 0 = stopped or not covered; plain sessions leave it 0).  A stopped pixel never starts
+// again, so an active pixel has taken exactly the samples 0 .. passes - 1, and in a plain session n_p = passes.
 // ------------------------------------------------------------------------------------------------------------
-// One sample pass of a session step, in place of k_sample_acc.  No k_store follows a step, so this counts the shadow
-// rays of every pass.
+struct AdaptParams {
+  uint32_t min_samples, max_samples;
+  float abs_error, rel_error;
+};
+
+// Sample fr.sample of the pixel at shard item k, from level-0 node `node`: S += c, Q += c c, n_p += 1, and the hit at
+// sample 0.  ADAPT: then the stop rule (crt_s_adapt_stop); returns true when it stops the pixel, whose flag it clears.
+template <bool ADAPT>
+CRT_DI bool accum_sample(const Frame &fr, const Levels &lv, uint32_t node, uint32_t k, const AdaptParams &ap,
+                         float4 *__restrict__ sum, float4 *__restrict__ sumsq, uint2 *__restrict__ hit0) {
+  const float4 c = lv.color[node], s = sum[k], q = sumsq[k];
+  const V3 a = vadd(mk(s.x, s.y, s.z), mk(c.x, c.y, c.z));
+  const V3 b = vadd(mk(q.x, q.y, q.z), mk(fmul(c.x, c.x), fmul(c.y, c.y), fmul(c.z, c.z)));
+  const uint32_t n = __float_as_uint(s.w) + 1u;
+  const float S[3] = {a.x, a.y, a.z}, Q[3] = {b.x, b.y, b.z};
+  const bool stop = ADAPT && crt_s_adapt_stop(n, S, Q, ap.min_samples, ap.max_samples, ap.abs_error, ap.rel_error) != 0;
+  sum[k] = make_float4(a.x, a.y, a.z, __uint_as_float(n));
+  sumsq[k] = make_float4(b.x, b.y, b.z, (ADAPT && !stop) ? 1.f : 0.f);
+  if (fr.sample == 0) hit0[k] = make_uint2(lv.hit_tri[node], __float_as_uint(lv.hit_t[node]));
+  return stop;
+}
+
+// One sample pass of a plain session step, in place of k_sample_acc.  No k_store follows a step, so this counts the
+// shadow rays of every pass.
 __global__ void __launch_bounds__(256) k_accum_step(const DScene sc, const Frame fr, const Levels lv, float4 *__restrict__ sum,
                                                    float4 *__restrict__ sumsq, uint2 *__restrict__ hit0) {
   if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&lv.stats[1], (unsigned long long)lv.counts[CRT_MAX_LEVELS] * sc.n_lights);
-  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x) {
-    const uint32_t node = lv.offset[0] + i, k = fr.item_begin + i;
-    const float4 c = lv.color[node], s = sum[k], q = sumsq[k];
-    const V3 a = vadd(mk(s.x, s.y, s.z), mk(c.x, c.y, c.z));
-    const V3 b = vadd(mk(q.x, q.y, q.z), mk(fmul(c.x, c.x), fmul(c.y, c.y), fmul(c.z, c.z)));
-    sum[k] = make_float4(a.x, a.y, a.z, 0.f);
-    sumsq[k] = make_float4(b.x, b.y, b.z, 0.f);
-    if (fr.sample == 0) hit0[k] = make_uint2(lv.hit_tri[node], __float_as_uint(lv.hit_t[node]));
-  }
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x)
+    accum_sample<false>(fr, lv, lv.offset[0] + i, fr.item_begin + i, AdaptParams{}, sum, sumsq, hit0);
 }
 
-// Read: S / float(n) (k_sample_acc's division) and the kept hit into the level-0 slots, for k_store
-__global__ void __launch_bounds__(256) k_accum_read(const Frame fr, const Levels lv, const float4 *__restrict__ sum,
-                                                   const uint2 *__restrict__ hit0, uint32_t n_samples) {
-  const float n = (float)n_samples;
-  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x) {
-    const uint32_t node = lv.offset[0] + i, k = fr.item_begin + i;
-    const float4 s = sum[k];
-    const uint2 h = hit0[k];
-    lv.color[node] = make_float4(fdiv(s.x, n), fdiv(s.y, n), fdiv(s.z, n), 0.f);
-    lv.hit_tri[node] = h.x;
-    lv.hit_t[node] = __uint_as_float(h.y);
-  }
+// The following kernels run once over a GPU's whole shard (item_begin 0).  Frame-layout arrays (H*W*3 floats, H*W hits
+// or counts) are in the primary's memory, peer-mapped on the other GPUs of a multi-GPU context, like k_store's frame.
+
+// Read: S / float(n_p) (k_sample_acc's division), its PPMColor bytes and the kept hit into the frame, stored as k_store
+// stores a frame
+__global__ void __launch_bounds__(256) k_accum_read(const DScene sc, const Frame fr, const float4 *__restrict__ sum,
+                                                   const uint2 *__restrict__ hit0, float *__restrict__ rgb,
+                                                   uint8_t *__restrict__ rgb8, HitRec *__restrict__ hits) {
+  store_items(
+      sc, fr, rgb, rgb8, hits, nullptr,
+      [&](uint32_t i) {
+        const float4 s = sum[fr.item_begin + i];
+        const float n = (float)__float_as_uint(s.w);
+        return make_float4(fdiv(s.x, n), fdiv(s.y, n), fdiv(s.z, n), 0.f);
+      },
+      [&](uint32_t i) {
+        const uint2 h = hit0[fr.item_begin + i];
+        HitRec r;
+        public_tri(sc, h.x, r);
+        r.t = h.x == CRT_INVALID ? 0.0f : __uint_as_float(h.y);
+        return r;
+      });
 }
 
-// Save: the accumulator of this chunk's covered pixels into frame-layout arrays (H*W*3 floats; public hit numbering,
-// mesh = triangle = -1 for a miss, t bits kept either way).  Any output may be null.
+// Save: the accumulator of the covered pixels into frame-layout arrays (public hit numbering, mesh = triangle = -1 for a
+// miss, t bits kept either way; counts = n_p).  Any output may be null.
 __global__ void __launch_bounds__(256) k_accum_save(const DScene sc, const Frame fr, const float4 *__restrict__ sum,
                                                    const float4 *__restrict__ sumsq, const uint2 *__restrict__ hit0,
                                                    float *__restrict__ sum_out, float *__restrict__ sumsq_out,
-                                                   HitRec *__restrict__ hit_out) {
+                                                   HitRec *__restrict__ hit_out, uint32_t *__restrict__ counts_out) {
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x) {
     uint32_t row, col;
     if (!item_pixel(fr, sc, fr.item_begin + i, row, col)) continue;
@@ -1611,60 +1651,80 @@ __global__ void __launch_bounds__(256) k_accum_save(const DScene sc, const Frame
     if (hit_out) {
       const uint2 h = hit0[k];
       HitRec r;
-      r.mesh = r.tri = -1;
-      if (h.x != CRT_INVALID) {
-        const uint32_t m = sc.tri_shade[h.x].w;
-        r.mesh = (int)m;
-        r.tri = (int)(h.x - sc.meshes[m].first_triangle);
-      }
+      public_tri(sc, h.x, r);
       r.t = __uint_as_float(h.y);
       hit_out[pix] = r;
     }
+    if (counts_out) counts_out[pix] = __float_as_uint(sum[k].w);
   }
 }
 
-// Load: the reverse of k_accum_save.  The hit records come from a file: one that names no triangle of the uploaded
-// scene sets *bad and is not used.
+// Load: the reverse of k_accum_save, or with sum_in == null (an adaptive begin) the counts and flags alone.  Per covered
+// pixel: S, Q and the hit from the inputs; n_p from counts_in, or `passes` without it; adaptive sessions set the
+// active flag iff n_p == passes and the rule does not stop the pixel at n_p.  The inputs come from a file: a hit record
+// that names no triangle of the uploaded scene sets bad[0], a count above passes or 0 while passes > 0 sets bad[1].
+// tot[0..2] += covered pixels, active pixels, sum of n_p.
 __global__ void __launch_bounds__(256) k_accum_load(const DScene sc, const Frame fr, const float *__restrict__ sum_in,
                                                    const float *__restrict__ sumsq_in, const HitRec *__restrict__ hit_in,
-                                                   uint32_t n_triangles, float4 *__restrict__ sum, float4 *__restrict__ sumsq,
-                                                   uint2 *__restrict__ hit0, uint32_t *__restrict__ bad) {
+                                                   const uint32_t *__restrict__ counts_in, uint32_t passes,
+                                                   uint32_t n_triangles, const bool adaptive, const AdaptParams ap,
+                                                   float4 *__restrict__ sum, float4 *__restrict__ sumsq,
+                                                   uint2 *__restrict__ hit0, uint32_t *__restrict__ bad,
+                                                   unsigned long long *__restrict__ tot) {
+  uint32_t covered = 0, active = 0;
+  unsigned long long samples = 0;
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x) {
     uint32_t row, col;
     if (!item_pixel(fr, sc, fr.item_begin + i, row, col)) continue;
     const uint32_t k = fr.item_begin + i;
     const size_t pix = (size_t)row * sc.width + col;
-    sum[k] = make_float4(sum_in[3 * pix + 0], sum_in[3 * pix + 1], sum_in[3 * pix + 2], 0.f);
-    sumsq[k] = make_float4(sumsq_in[3 * pix + 0], sumsq_in[3 * pix + 1], sumsq_in[3 * pix + 2], 0.f);
-    const HitRec r = hit_in[pix];
-    uint32_t tri = CRT_INVALID;
-    if (r.mesh >= 0) {
-      const bool ok = (uint32_t)r.mesh < sc.n_meshes && r.tri >= 0 &&
-                      (unsigned long long)sc.meshes[r.mesh].first_triangle + (uint32_t)r.tri < n_triangles &&
-                      sc.tri_shade[sc.meshes[r.mesh].first_triangle + (uint32_t)r.tri].w == (uint32_t)r.mesh;
-      if (!ok) {
-        *bad = 1u;
+    float4 s = sum[k], q = sumsq[k];
+    if (sum_in) {
+      s = make_float4(sum_in[3 * pix + 0], sum_in[3 * pix + 1], sum_in[3 * pix + 2], 0.f);
+      q = make_float4(sumsq_in[3 * pix + 0], sumsq_in[3 * pix + 1], sumsq_in[3 * pix + 2], 0.f);
+      const HitRec r = hit_in[pix];
+      uint32_t tri = CRT_INVALID;
+      if (r.mesh >= 0) {
+        const bool ok = (uint32_t)r.mesh < sc.n_meshes && r.tri >= 0 &&
+                        (unsigned long long)sc.meshes[r.mesh].first_triangle + (uint32_t)r.tri < n_triangles &&
+                        sc.tri_shade[sc.meshes[r.mesh].first_triangle + (uint32_t)r.tri].w == (uint32_t)r.mesh;
+        if (!ok) {
+          bad[0] = 1u;
+          continue;
+        }
+        tri = sc.meshes[r.mesh].first_triangle + (uint32_t)r.tri;
+      } else if (r.mesh != -1 || r.tri != -1) {
+        bad[0] = 1u;
         continue;
       }
-      tri = sc.meshes[r.mesh].first_triangle + (uint32_t)r.tri;
-    } else if (r.mesh != -1 || r.tri != -1) {
-      *bad = 1u;
+      hit0[k] = make_uint2(tri, __float_as_uint(r.t));
+    }
+    const uint32_t n = counts_in ? counts_in[pix] : passes;
+    if (n > passes || (n == 0 && passes > 0)) {
+      bad[1] = 1u;
       continue;
     }
-    hit0[k] = make_uint2(tri, __float_as_uint(r.t));
+    const float S[3] = {s.x, s.y, s.z}, Q[3] = {q.x, q.y, q.z};
+    const bool act = adaptive && n == passes && !crt_s_adapt_stop(n, S, Q, ap.min_samples, ap.max_samples, ap.abs_error, ap.rel_error);
+    sum[k] = make_float4(s.x, s.y, s.z, __uint_as_float(n));
+    sumsq[k] = make_float4(q.x, q.y, q.z, act ? 1.f : 0.f);
+    covered++;
+    active += act ? 1u : 0u;
+    samples += n;
+  }
+  covered = __reduce_add_sync(CRT_FULL_MASK, covered);
+  active = __reduce_add_sync(CRT_FULL_MASK, active);
+  for (int d = 16; d > 0; d >>= 1) samples += __shfl_xor_sync(CRT_FULL_MASK, samples, d);
+  if (lane_id() == 0 && covered) {
+    atomicAdd(&tot[0], (unsigned long long)covered);
+    atomicAdd(&tot[1], (unsigned long long)active);
+    atomicAdd(&tot[2], samples);
   }
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// Adaptive sessions (crtb200_accum_begin_adaptive, DESIGN.md 3.10.2).  Same accumulator; its unused w lanes hold the
-// pixel's sample count n_p (S.w, as uint32 bits) and its active flag (Q.w: 1 = still sampling, 0 = stopped or not
-// covered).  A stopped pixel never starts again, so an active pixel has taken exactly the samples 0 .. passes - 1.
+// Adaptive session passes (crtb200_accum_begin_adaptive, DESIGN.md 3.10.2)
 // ------------------------------------------------------------------------------------------------------------
-struct AdaptParams {
-  uint32_t min_samples, max_samples;
-  float abs_error, rel_error;
-};
-
 // Per pass and chunk: the shard items still sampling, into list[0 .. *n_list) (*n_list zeroed before).  One warp per
 // 8x4 tile, one ballot and one atomicAdd, so a tile's active pixels stay adjacent and a level-0 warp starts coherent.
 // The order of tiles in the list varies from run to run; nothing depends on it (path keys follow the ray's place in
@@ -1684,9 +1744,8 @@ __global__ void __launch_bounds__(256) k_adapt_compact(const Frame fr, const flo
   }
 }
 
-// One adaptive pass, in place of k_accum_step: S += c, Q += c c, n_p += 1 at shard item list[j], the hit at sample 0,
-// then the stop rule (crt_s_adapt_stop) clears the active flag.  Counts the pass's shadow rays as k_accum_step does,
-// its pixel-samples into stats[42] and the pixels it stopped into stats[43].
+// One adaptive pass, in place of k_accum_step: accum_sample with the stop rule at shard item list[j].  Counts the
+// pass's shadow rays as k_accum_step does, its pixel-samples into stats[42] and the pixels it stopped into stats[43].
 __global__ void __launch_bounds__(256) k_adapt_step(const DScene sc, const Frame fr, const Levels lv, const AdaptParams ap,
                                                    float4 *__restrict__ sum, float4 *__restrict__ sumsq,
                                                    uint2 *__restrict__ hit0) {
@@ -1698,83 +1757,9 @@ __global__ void __launch_bounds__(256) k_adapt_step(const DScene sc, const Frame
   const uint32_t stride = gridDim.x * blockDim.x;
   for (uint32_t base = blockIdx.x * blockDim.x + (threadIdx.x & ~31u); base < n_act; base += stride) {
     const uint32_t j = base + lane_id();
-    bool stop = false;
-    if (j < n_act) {
-      const uint32_t node = lv.offset[0] + j, k = fr.list[j];
-      const float4 c = lv.color[node], s = sum[k], q = sumsq[k];
-      const V3 a = vadd(mk(s.x, s.y, s.z), mk(c.x, c.y, c.z));
-      const V3 b = vadd(mk(q.x, q.y, q.z), mk(fmul(c.x, c.x), fmul(c.y, c.y), fmul(c.z, c.z)));
-      const uint32_t n = __float_as_uint(s.w) + 1u;
-      const float S[3] = {a.x, a.y, a.z}, Q[3] = {b.x, b.y, b.z};
-      stop = crt_s_adapt_stop(n, S, Q, ap.min_samples, ap.max_samples, ap.abs_error, ap.rel_error) != 0;
-      sum[k] = make_float4(a.x, a.y, a.z, __uint_as_float(n));
-      sumsq[k] = make_float4(b.x, b.y, b.z, stop ? 0.f : 1.f);
-      if (fr.sample == 0) hit0[k] = make_uint2(lv.hit_tri[node], __float_as_uint(lv.hit_t[node]));
-    }
+    const bool stop = j < n_act && accum_sample<true>(fr, lv, lv.offset[0] + j, fr.list[j], ap, sum, sumsq, hit0);
     const uint32_t stopped = __popc(__ballot_sync(CRT_FULL_MASK, stop));
     if (lane_id() == 0 && stopped) atomicAdd(&lv.stats[43], (unsigned long long)stopped);
-  }
-}
-
-// Read: S / float(n_p) and the kept hit into the level-0 slots, for k_store (k_accum_read with the pixel's own count)
-__global__ void __launch_bounds__(256) k_adapt_read(const Frame fr, const Levels lv, const float4 *__restrict__ sum,
-                                                   const uint2 *__restrict__ hit0) {
-  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x) {
-    const uint32_t node = lv.offset[0] + i, k = fr.item_begin + i;
-    const float4 s = sum[k];
-    const uint2 h = hit0[k];
-    const float n = (float)__float_as_uint(s.w);
-    lv.color[node] = make_float4(fdiv(s.x, n), fdiv(s.y, n), fdiv(s.z, n), 0.f);
-    lv.hit_tri[node] = h.x;
-    lv.hit_t[node] = __uint_as_float(h.y);
-  }
-}
-
-// Counts and flags of the covered pixels after begin (counts_in null, passes 0) or a load (behind k_accum_load, which
-// zeroes the w lanes).  counts_in: H*W frame-layout counts, or null for n_p = passes everywhere.  A pixel is active iff
-// n_p == passes and the rule does not stop it at n_p; a count above passes, or 0 while passes > 0, sets *bad.
-// tot[0..2] += covered pixels, active pixels, sum of n_p.
-__global__ void __launch_bounds__(256) k_adapt_counts(const DScene sc, const Frame fr, const uint32_t *__restrict__ counts_in,
-                                                     uint32_t passes, const AdaptParams ap, float4 *__restrict__ sum,
-                                                     float4 *__restrict__ sumsq, uint32_t *__restrict__ bad,
-                                                     unsigned long long *__restrict__ tot) {
-  uint32_t covered = 0, active = 0;
-  unsigned long long samples = 0;
-  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x) {
-    uint32_t row, col;
-    if (!item_pixel(fr, sc, fr.item_begin + i, row, col)) continue;
-    const uint32_t k = fr.item_begin + i;
-    const uint32_t n = counts_in ? counts_in[(size_t)row * sc.width + col] : passes;
-    if (n > passes || (n == 0 && passes > 0)) {
-      *bad = 1u;
-      continue;
-    }
-    const float4 s = sum[k], q = sumsq[k];
-    const float S[3] = {s.x, s.y, s.z}, Q[3] = {q.x, q.y, q.z};
-    const bool act = n == passes && !crt_s_adapt_stop(n, S, Q, ap.min_samples, ap.max_samples, ap.abs_error, ap.rel_error);
-    sum[k].w = __uint_as_float(n);
-    sumsq[k].w = act ? 1.f : 0.f;
-    covered++;
-    active += act ? 1u : 0u;
-    samples += n;
-  }
-  covered = __reduce_add_sync(CRT_FULL_MASK, covered);
-  active = __reduce_add_sync(CRT_FULL_MASK, active);
-  for (int d = 16; d > 0; d >>= 1) samples += __shfl_xor_sync(CRT_FULL_MASK, samples, d);
-  if (lane_id() == 0 && covered) {
-    atomicAdd(&tot[0], (unsigned long long)covered);
-    atomicAdd(&tot[1], (unsigned long long)active);
-    atomicAdd(&tot[2], samples);
-  }
-}
-
-// Save of the counts map: n_p of the covered pixels into H*W frame-layout counts (the caller zeroes the rest)
-__global__ void __launch_bounds__(256) k_adapt_save(const DScene sc, const Frame fr, const float4 *__restrict__ sum,
-                                                   uint32_t *__restrict__ counts_out) {
-  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x) {
-    uint32_t row, col;
-    if (!item_pixel(fr, sc, fr.item_begin + i, row, col)) continue;
-    counts_out[(size_t)row * sc.width + col] = __float_as_uint(sum[fr.item_begin + i].w);
   }
 }
 
@@ -1901,16 +1886,8 @@ __global__ void __launch_bounds__(256) k_query(const DScene sc, const float *__r
         }
       }
       HitRec h;
-      if (cl.best_tri == CRT_INVALID) {
-        h.mesh = -1;
-        h.tri = -1;
-        h.t = 0.0f;
-      } else {
-        const uint32_t m = sc.tri_shade[cl.best_tri].w;
-        h.mesh = (int)m;
-        h.tri = (int)(cl.best_tri - sc.meshes[m].first_triangle);
-        h.t = cl.best_t;
-      }
+      public_tri(sc, cl.best_tri, h);
+      h.t = cl.best_tri == CRT_INVALID ? 0.0f : cl.best_t;
       hits[i] = h;
     }
   }

@@ -1531,24 +1531,19 @@ struct HostOut {
   crtb200_hit *hits = nullptr;
 };
 
-// A pass of a progressive session (DESIGN.md 3.10.1) through the chunk loop of enqueue_frame, on the accumulator of the
-// context it runs on.  STEP renders global samples [s0, s0 + n) into it; READ stores S / float(s0) and the kept hit
-// through k_store; SAVE / LOAD move it to / from frame-layout arrays in the primary's memory (peer-mapped on the other
-// GPUs of a multi-GPU context, like k_store's frame).  No pass but STEP runs a sample.
+// A step of a progressive session (DESIGN.md 3.10.1): global samples [s0, s0 + n) through the chunk loop of
+// enqueue_frame, into the accumulator of the context it runs on.  ap: the stop rule of an adaptive session (DESIGN.md
+// 3.10.2), whose passes compact the active pixels before each sample and run k_adapt_step; null for a plain session.
 struct AccumPass {
-  enum Mode { STEP, READ, SAVE, LOAD, COUNTS } mode;
   uint32_t s0, n;
-  float *px_sum, *px_sumsq;
-  HitRec *px_hit;
-  uint32_t *bad;  // LOAD: set when a hit record names no triangle of the scene (or, adaptive, a count is out of range)
-  // adaptive sessions (DESIGN.md 3.10.2): STEP compacts the active pixels before each sample and runs k_adapt_step;
-  // READ divides by each pixel's own count; SAVE also writes px_counts (if not null); COUNTS sets the counts (px_counts,
-  // null: every count is s0) and the flags, and adds covered pixels, active pixels and pixel-samples into tot[0..2].
-  bool adaptive;
-  AdaptParams ap;
-  uint32_t *px_counts;
-  unsigned long long *tot;
+  const AdaptParams *ap;
 };
+
+// level-0 work items of tile shard `index` of `count`: 8x4-pixel tiles dealt round-robin, 32 items each
+static uint32_t shard_item_count(const crtb200_ctx *c, uint32_t index, uint32_t count) {
+  const uint32_t tiles = ((c->sc.width + 7) / 8) * ((c->sc.height + 3) / 4);
+  return (tiles > index ? (tiles - index + count - 1) / count : 0) * 32u;
+}
 
 // Enqueue one frame on `st`.  d_rgb / d_rgb8 / d_hits / d_slab are device pointers (any may be null).
 static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_options *o, float *d_rgb,
@@ -1590,8 +1585,7 @@ static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb20
   fr.seed = c->sampling.seed;
   fr.frame_index = c->sampling.frame_index + c->frame_offset;
   fr.mc_bias = c->sampling.monte_carlo_bias;
-  const uint32_t shard_tiles = (fr.n_tiles > o->shard_index) ? (fr.n_tiles - o->shard_index + shard_count - 1) / shard_count : 0;
-  const uint32_t shard_items = shard_tiles * 32u;
+  const uint32_t shard_items = shard_item_count(c, o->shard_index, shard_count);
   // unsharded frames: chunks are whole rows of tiles, so a chunk owns a contiguous band of image rows
   const uint32_t row_items = (shard_count == 1) ? fr.tiles_x * 32u : 32u;
   rc = plan_queues(c, std::max(shard_items, 32u), o->max_depth, row_items, host != nullptr);
@@ -1643,7 +1637,7 @@ static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb20
       CUDA_TRY(q.acc.ensure(c->cap_items));
       CUDA_TRY(q.hit0.ensure(c->cap_items));
     }
-    const bool adapt_step = acc && acc->adaptive && acc->mode == AccumPass::STEP;
+    const bool adapt_step = acc && acc->ap;
     if (adapt_step) {
       CUDA_TRY(q.alist.ensure(c->cap_items));
       CUDA_TRY(q.acount.ensure(1));
@@ -1735,7 +1729,7 @@ static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb20
         launches++;
       }
       if (adapt_step) {
-        k_adapt_step<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, acc->ap, c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p);
+        k_adapt_step<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, *acc->ap, c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p);
         launches++;
       } else if (acc) {
         k_accum_step<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p);
@@ -1745,32 +1739,7 @@ static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb20
         launches++;
       }
     }
-    fr.list = fr.n_list = nullptr;
-    if (acc && acc->mode == AccumPass::READ) {
-      CUDA_TRY(cudaMemsetAsync(q.ctl.p, 0, q.ctl.n * sizeof(uint32_t), qs));  // k_store then counts no shadow rays
-      if (acc->adaptive)
-        k_adapt_read<<<grid_simple, 256, 0, qs>>>(fr, q.lv, c->acc_sum.p, c->acc_hit.p);
-      else
-        k_accum_read<<<grid_simple, 256, 0, qs>>>(fr, q.lv, c->acc_sum.p, c->acc_hit.p, acc->s0);
-      launches++;
-    } else if (acc && acc->mode == AccumPass::SAVE) {
-      k_accum_save<<<grid_simple, 256, 0, qs>>>(c->sc, fr, c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p, acc->px_sum,
-                                                acc->px_sumsq, acc->px_hit);
-      launches++;
-      if (acc->px_counts) {
-        k_adapt_save<<<grid_simple, 256, 0, qs>>>(c->sc, fr, c->acc_sum.p, acc->px_counts);
-        launches++;
-      }
-    } else if (acc && acc->mode == AccumPass::LOAD) {
-      k_accum_load<<<grid_simple, 256, 0, qs>>>(c->sc, fr, acc->px_sum, acc->px_sumsq, acc->px_hit, c->n_triangles,
-                                                c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p, acc->bad);
-      launches++;
-    } else if (acc && acc->mode == AccumPass::COUNTS) {
-      k_adapt_counts<<<grid_simple, 256, 0, qs>>>(c->sc, fr, acc->px_counts, acc->s0, acc->ap, c->acc_sum.p, c->acc_sumsq.p,
-                                                  acc->bad, acc->tot);
-      launches++;
-    }
-    if (!acc || acc->mode == AccumPass::READ) {
+    if (!acc) {
       k_store<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, d_rgb, d_rgb8, d_hits, d_slab);
       launches++;
     }
@@ -2136,22 +2105,36 @@ int crtb200_render_device(crtb200_ctx *c, const crtb200_camera *cam, const crtb2
 }
 
 // ---- progressive sessions (DESIGN.md 3.10.1) ---------------------------------------------------------------------
-// One session pass on every GPU of the context, with the session's snapshots.  The session's sampling stands in for the
-// context's for the call, because queue planning and the Philox key both read ctx->sampling; frame_offset is 0 outside
-// crtb200_render_frames, so the key is the session's frame_index.
-static int session_pass(crtb200_ctx *c, const AccumPass &a, float *d_rgb, uint8_t *d_rgb8, HitRec *d_hits, bool timed) {
-  std::vector<crtb200_sampling> saved;
-  for (size_t i = 0; i <= c->peers.size(); i++) {
+// One kernel over the whole tile shard of every GPU of the context: Frame with item_begin 0 and the session's rects;
+// launch(x, fr, stream) enqueues GPU x's kernel.  Queues, device counters, the last render's statistics and the
+// context's sampling stay as they are.  As in enqueue_any, the peers start after c->stream has reached this point and
+// c->stream continues after every peer's kernel.
+static int shard_pass(crtb200_ctx *c, const std::function<void(crtb200_ctx *, const Frame &, cudaStream_t)> &launch) {
+  const uint32_t n = 1u + (uint32_t)c->peers.size();
+  if (n > 1) CUDA_TRY(cudaEventRecord(c->multi_fork, c->stream));
+  for (uint32_t i = 0; i < n; i++) {
     crtb200_ctx *x = i ? c->peers[i - 1] : c;
-    saved.push_back(x->sampling);
-    x->sampling = c->acc_smp;
+    CUDA_TRY(cudaSetDevice(x->device));
+    const int rc = plan_mask(x, &c->acc_opt);
+    if (rc) return rc;
+    Frame fr{};
+    fr.tiles_x = (x->sc.width + 7) / 8;
+    fr.n_tiles = fr.tiles_x * ((x->sc.height + 3) / 4);
+    fr.shard_index = i;
+    fr.shard_count = n;
+    fr.mask = x->mask_needed ? x->mask.p : nullptr;
+    fr.n_items0 = shard_item_count(x, i, n);
+    if (i) CUDA_TRY(cudaStreamWaitEvent(x->stream, c->multi_fork, 0));
+    launch(x, fr, x->stream);
+    CUDA_TRY(cudaGetLastError());
+    if (i) CUDA_TRY(cudaEventRecord(x->multi_done, x->stream));
   }
-  const int rc = enqueue_any(c, &c->acc_cam, &c->acc_opt, d_rgb, d_rgb8, d_hits, nullptr, c->stream, timed, nullptr, nullptr, false, &a);
-  for (size_t i = 0; i <= c->peers.size(); i++) (i ? c->peers[i - 1] : c)->sampling = saved[i];
-  return rc;
+  CUDA_TRY(cudaSetDevice(c->device));
+  for (crtb200_ctx *p : c->peers) CUDA_TRY(cudaStreamWaitEvent(c->stream, p->multi_done, 0));
+  return CRTB200_OK;
 }
 
-// device staging of a save / load: frame-layout S, Q and hit records on the primary
+// device staging of a save / load: frame-layout S, Q, hit records and counts on the primary
 struct AccumStaging {
   DevBuf<float> sum, sumsq;
   DevBuf<HitRec> hit;
@@ -2167,24 +2150,29 @@ struct AccumStaging {
   }
 };
 
-// The session pass that sets an adaptive session's counts and flags: after begin (passes 0) or behind a load's
-// k_accum_load (g.counts empty = passes everywhere).  g.tot (zeroed by the caller) receives the totals the session
-// keeps on the host; g.bad, when allocated, any out-of-range count.
-static int accum_counts_pass(crtb200_ctx *c, uint32_t passes, AccumStaging &g) {
-  const crtb200_stats keep = c->last;
-  const uint32_t keep_samples = c->last_samples;
-  AccumPass a{AccumPass::COUNTS, passes, 0, nullptr, nullptr, nullptr, g.bad.p};
-  a.adaptive = true;
-  a.ap = c->acc_ap;
-  a.px_counts = g.counts.p;
-  a.tot = g.tot.p;
-  const int rc = session_pass(c, a, nullptr, nullptr, nullptr, false);
-  c->last = keep;
-  c->last_samples = keep_samples;
+// k_accum_load on every GPU from the staged arrays (all empty: an adaptive begin's flags), then the totals the session
+// keeps on the host.  Inputs that do not fit the scene or `passes` end the session.
+static int accum_load_pass(crtb200_ctx *c, AccumStaging &g, uint32_t passes) {
+  CUDA_TRY(g.bad.ensure(2));
+  CUDA_TRY(g.tot.ensure(3));
+  CUDA_TRY(cudaMemsetAsync(g.bad.p, 0, 2 * sizeof(uint32_t), c->stream));
+  CUDA_TRY(cudaMemsetAsync(g.tot.p, 0, 3 * sizeof(unsigned long long), c->stream));
+  const int rc = shard_pass(c, [&](crtb200_ctx *x, const Frame &fr, cudaStream_t st) {
+    k_accum_load<<<x->sm_count * 8, 256, 0, st>>>(x->sc, fr, g.sum.p, g.sumsq.p, g.hit.p, g.counts.p, passes, x->n_triangles,
+                                                  c->acc_adaptive, c->acc_ap, x->acc_sum.p, x->acc_sumsq.p, x->acc_hit.p,
+                                                  g.bad.p, g.tot.p);
+  });
   if (rc) return rc;
+  uint32_t bad[2];
   unsigned long long tot[3];
+  CUDA_TRY(cudaMemcpyAsync(bad, g.bad.p, sizeof(bad), cudaMemcpyDeviceToHost, c->stream));
   CUDA_TRY(cudaMemcpyAsync(tot, g.tot.p, sizeof(tot), cudaMemcpyDeviceToHost, c->stream));
   CUDA_TRY(cudaStreamSynchronize(c->stream));
+  if (bad[0] || bad[1]) {
+    accum_release(c);
+    return fail(CRTB200_ERR_ARG, bad[0] ? "hit records name triangles the uploaded scene does not have; the session has ended"
+                                        : "a count exceeds passes, or is 0 inside the rects while passes > 0; the session has ended");
+  }
   c->acc_covered = tot[0];
   c->acc_active_px = tot[1];
   c->acc_px_samples = tot[2];
@@ -2216,10 +2204,9 @@ static int accum_begin(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_
   c->acc_smp.use_gi = 1;
   c->acc_smp.rays_per_pixel = 1;  // unused: a step says how many samples it renders
   const uint32_t n = 1u + (uint32_t)c->peers.size();
-  const uint32_t tiles = ((c->sc.width + 7) / 8) * ((c->sc.height + 3) / 4);
   for (uint32_t i = 0; i < n; i++) {
     crtb200_ctx *x = i ? c->peers[i - 1] : c;
-    const size_t items = std::max<size_t>(1, (size_t)(tiles > i ? (tiles - i + n - 1) / n : 0) * 32u);  // shard i of n
+    const size_t items = std::max<size_t>(1, shard_item_count(c, i, n));
     cudaError_t e = cudaSetDevice(x->device);
     if (e == cudaSuccess) e = x->acc_sum.ensure(items);
     if (e == cudaSuccess) e = x->acc_sumsq.ensure(items);
@@ -2246,14 +2233,9 @@ static int accum_begin(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_
   c->acc_ap = AdaptParams{ad->min_samples, ad->max_samples, ad->abs_error, ad->rel_error};
   // every covered pixel starts active: the flags are set on the device, shard by shard
   AccumStaging g;
-  CUDA_TRY(g.tot.ensure(3));
-  CUDA_TRY(cudaMemsetAsync(g.tot.p, 0, 3 * sizeof(unsigned long long), c->stream));
-  const int rc = accum_counts_pass(c, 0, g);
-  if (rc) {
-    accum_release(c);
-    return rc;
-  }
-  return CRTB200_OK;
+  const int rc = accum_load_pass(c, g, 0);
+  if (rc) accum_release(c);
+  return rc;
 }
 
 int crtb200_accum_begin(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_options *o, const crtb200_sampling *s) {
@@ -2276,10 +2258,17 @@ int crtb200_accum_step(crtb200_ctx *c, uint32_t n_samples, crtb200_stats *stats)
   if (n_samples == 0 || (uint64_t)c->acc_done + n_samples > 0xFFFFFFFFull) return fail(CRTB200_ERR_ARG, "n_samples must be at least 1");
   const auto t0 = std::chrono::steady_clock::now();
   c->last = crtb200_stats{};
-  AccumPass a{AccumPass::STEP, c->acc_done, n_samples, nullptr, nullptr, nullptr, nullptr};
-  a.adaptive = c->acc_adaptive;
-  a.ap = c->acc_ap;
-  int rc = session_pass(c, a, nullptr, nullptr, nullptr, true);
+  const AccumPass a{c->acc_done, n_samples, c->acc_adaptive ? &c->acc_ap : nullptr};
+  // The session's sampling stands in for the context's during the step, because queue planning and the Philox key both
+  // read ctx->sampling; frame_offset is 0 outside crtb200_render_frames, so the key is the session's frame_index.
+  std::vector<crtb200_sampling> saved;
+  for (size_t i = 0; i <= c->peers.size(); i++) {
+    crtb200_ctx *x = i ? c->peers[i - 1] : c;
+    saved.push_back(x->sampling);
+    x->sampling = c->acc_smp;
+  }
+  int rc = enqueue_any(c, &c->acc_cam, &c->acc_opt, nullptr, nullptr, nullptr, nullptr, c->stream, true, nullptr, nullptr, false, &a);
+  for (size_t i = 0; i <= c->peers.size(); i++) (i ? c->peers[i - 1] : c)->sampling = saved[i];
   if (rc) return rc;
   CUDA_TRY(cudaStreamSynchronize(c->stream));
   rc = collect_stats(c, true);
@@ -2303,14 +2292,10 @@ int crtb200_accum_read(crtb200_ctx *c, float *rgb_out, uint8_t *rgb8_out, crtb20
   const size_t px = (size_t)c->sc.width * c->sc.height;
   if (hits_out) CUDA_TRY(c->hits.ensure(px));
   if (hits_out) CUDA_TRY(cudaMemsetAsync(c->hits.p, 0xFF, px * sizeof(HitRec), c->stream));
-  // a read is no render: the last render's statistics stay what they were
-  const crtb200_stats keep = c->last;
-  const uint32_t keep_samples = c->last_samples;
-  AccumPass a{AccumPass::READ, c->acc_done, 0, nullptr, nullptr, nullptr, nullptr};
-  a.adaptive = c->acc_adaptive;
-  const int rc = session_pass(c, a, c->frame.p, rgb8_out ? c->frame8.p : nullptr, hits_out ? c->hits.p : nullptr, false);
-  c->last = keep;
-  c->last_samples = keep_samples;
+  const int rc = shard_pass(c, [&](crtb200_ctx *x, const Frame &fr, cudaStream_t st) {
+    k_accum_read<<<x->sm_count * 8, 256, 0, st>>>(x->sc, fr, x->acc_sum.p, x->acc_hit.p, c->frame.p,
+                                                  rgb8_out ? c->frame8.p : nullptr, hits_out ? c->hits.p : nullptr);
+  });
   if (rc) return rc;
   if (rgb_out) CUDA_TRY(cudaMemcpyAsync(rgb_out, c->frame.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
   if (rgb8_out) CUDA_TRY(cudaMemcpyAsync(rgb8_out, c->frame8.p, px * 3, cudaMemcpyDeviceToHost, c->stream));
@@ -2318,6 +2303,14 @@ int crtb200_accum_read(crtb200_ctx *c, float *rgb_out, uint8_t *rgb8_out, crtb20
   CUDA_TRY(cudaStreamSynchronize(c->stream));
   if (samples_done) *samples_done = c->acc_done;
   return CRTB200_OK;
+}
+
+// k_accum_save on every GPU into the staged arrays (any may be empty)
+static int accum_save_pass(crtb200_ctx *c, AccumStaging &g) {
+  return shard_pass(c, [&](crtb200_ctx *x, const Frame &fr, cudaStream_t st) {
+    k_accum_save<<<x->sm_count * 8, 256, 0, st>>>(x->sc, fr, x->acc_sum.p, x->acc_sumsq.p, x->acc_hit.p, g.sum.p, g.sumsq.p,
+                                                  g.hit.p, g.counts.p);
+  });
 }
 
 int crtb200_accum_save(crtb200_ctx *c, float *sum_out, float *sumsq_out, crtb200_hit *hit0_out, uint32_t *samples_done) {
@@ -2339,12 +2332,7 @@ int crtb200_accum_save(crtb200_ctx *c, float *sum_out, float *sumsq_out, crtb200
     CUDA_TRY(g.hit.ensure(px));
     CUDA_TRY(cudaMemsetAsync(g.hit.p, 0xFF, px * sizeof(HitRec), c->stream));
   }
-  const crtb200_stats keep = c->last;
-  const uint32_t keep_samples = c->last_samples;
-  const AccumPass a{AccumPass::SAVE, c->acc_done, 0, g.sum.p, g.sumsq.p, g.hit.p, nullptr};
-  const int rc = session_pass(c, a, nullptr, nullptr, nullptr, false);
-  c->last = keep;
-  c->last_samples = keep_samples;
+  const int rc = accum_save_pass(c, g);
   if (rc) return rc;
   if (sum_out) CUDA_TRY(cudaMemcpyAsync(sum_out, g.sum.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
   if (sumsq_out) CUDA_TRY(cudaMemcpyAsync(sumsq_out, g.sumsq.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
@@ -2366,42 +2354,16 @@ static int accum_load(crtb200_ctx *c, const float *sum, const float *sumsq, cons
   CUDA_TRY(g.sum.ensure(px * 3));
   CUDA_TRY(g.sumsq.ensure(px * 3));
   CUDA_TRY(g.hit.ensure(px));
-  CUDA_TRY(g.bad.ensure(1));
   CUDA_TRY(cudaMemcpyAsync(g.sum.p, sum, px * 3 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
   CUDA_TRY(cudaMemcpyAsync(g.sumsq.p, sumsq, px * 3 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
   CUDA_TRY(cudaMemcpyAsync(g.hit.p, hit0, px * sizeof(HitRec), cudaMemcpyHostToDevice, c->stream));
-  CUDA_TRY(cudaMemsetAsync(g.bad.p, 0, sizeof(uint32_t), c->stream));
-  const crtb200_stats keep = c->last;
-  const uint32_t keep_samples = c->last_samples;
-  const AccumPass a{AccumPass::LOAD, 0, 0, g.sum.p, g.sumsq.p, g.hit.p, g.bad.p};
-  int rc = session_pass(c, a, nullptr, nullptr, nullptr, false);
-  c->last = keep;
-  c->last_samples = keep_samples;
-  if (rc) return rc;
-  uint32_t bad = 0;
-  CUDA_TRY(cudaMemcpyAsync(&bad, g.bad.p, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
-  CUDA_TRY(cudaStreamSynchronize(c->stream));
-  if (bad) {
-    accum_release(c);
-    return fail(CRTB200_ERR_ARG, "hit records name triangles the uploaded scene does not have; the session has ended");
-  }
-  c->acc_done = samples_done;
-  if (!c->acc_adaptive) return CRTB200_OK;
-  // the counts and flags, behind k_accum_load (which zeroed them) on the same streams
   if (counts) {
     CUDA_TRY(g.counts.ensure(px));
     CUDA_TRY(cudaMemcpyAsync(g.counts.p, counts, px * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
   }
-  CUDA_TRY(g.tot.ensure(3));
-  CUDA_TRY(cudaMemsetAsync(g.tot.p, 0, 3 * sizeof(unsigned long long), c->stream));
-  rc = accum_counts_pass(c, samples_done, g);
+  const int rc = accum_load_pass(c, g, samples_done);
   if (rc) return rc;
-  CUDA_TRY(cudaMemcpyAsync(&bad, g.bad.p, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
-  CUDA_TRY(cudaStreamSynchronize(c->stream));
-  if (bad) {
-    accum_release(c);
-    return fail(CRTB200_ERR_ARG, "a count exceeds passes, or is 0 inside the rects while passes > 0; the session has ended");
-  }
+  c->acc_done = samples_done;
   return CRTB200_OK;
 }
 
@@ -2434,27 +2396,10 @@ int crtb200_accum_counts(crtb200_ctx *c, uint32_t *counts_out) {
   CUDA_TRY(cudaSetDevice(c->device));
   if (!c->acc_active) return fail(CRTB200_ERR_STATE, "no progressive session (crtb200_accum_begin)");
   const size_t px = (size_t)c->sc.width * c->sc.height;
-  if (!c->acc_adaptive) {  // every covered pixel has taken every pass
-    if (c->acc_rects.empty()) {
-      std::fill(counts_out, counts_out + px, c->acc_done);
-    } else {
-      std::vector<uint8_t> m;
-      rect_coverage(c->sc.width, c->sc.height, c->acc_rects, m);
-      for (size_t i = 0; i < px; i++) counts_out[i] = m[i] ? c->acc_done : 0u;
-    }
-    return CRTB200_OK;
-  }
   AccumStaging g;
   CUDA_TRY(g.counts.ensure(px));
   CUDA_TRY(cudaMemsetAsync(g.counts.p, 0, px * sizeof(uint32_t), c->stream));
-  const crtb200_stats keep = c->last;
-  const uint32_t keep_samples = c->last_samples;
-  AccumPass a{AccumPass::SAVE, c->acc_done, 0, nullptr, nullptr, nullptr, nullptr};
-  a.adaptive = true;
-  a.px_counts = g.counts.p;
-  const int rc = session_pass(c, a, nullptr, nullptr, nullptr, false);
-  c->last = keep;
-  c->last_samples = keep_samples;
+  const int rc = accum_save_pass(c, g);
   if (rc) return rc;
   CUDA_TRY(cudaMemcpyAsync(counts_out, g.counts.p, px * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
   CUDA_TRY(cudaStreamSynchronize(c->stream));
@@ -2487,8 +2432,7 @@ int crtb200_shard_items(crtb200_ctx *c, uint32_t shard_count, uint32_t *items) {
   ErrScope scope(c);
   if (!c || !items || shard_count == 0) return fail(CRTB200_ERR_ARG, "bad argument");
   if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
-  const uint32_t tiles = ((c->sc.width + 7) / 8) * ((c->sc.height + 3) / 4);
-  *items = ((tiles + shard_count - 1) / shard_count) * 32u;
+  *items = shard_item_count(c, 0, shard_count);  // shard 0 is the largest
   return CRTB200_OK;
 }
 
