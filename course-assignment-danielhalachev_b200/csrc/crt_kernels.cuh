@@ -64,7 +64,7 @@ struct Levels {
   float4 *dq;         // diffuse queue, 3 x float4 per item: {P, bits(node)} {N, base.r} {base.g, base.b, -, -}
   uint8_t *vis;       // per (diffuse item, light): 1 = the light is visible from the hit
   uint32_t *counts;   // [CRT_MAX_LEVELS] rays per level; [CRT_MAX_LEVELS] = diffuse queue length
-  unsigned long long *stats;  // [0..3] rays by type, [4],[5] closest node / triangle tests, [6],[7] shadow, [32],[33] walks handed to k_coop, [40] shadow rays answered without a walk, [41] diffuse rays
+  unsigned long long *stats;  // device counters of the frame, CRT_STAT_SLOTS of them (named below)
   uint32_t offset[CRT_MAX_LEVELS + 1];
   // tail hand-off (k_coop): once the work queue of a traversal kernel is dry, the walks still running are written to
   // ovf[] (3 x uint4 per record) and finished one WARP per ray; tail_iters = 0 switches this off
@@ -78,6 +78,19 @@ struct Levels {
   uint32_t tail_start_closest;  // ... closest-hit launches
   uint32_t tail_small;  // launches of at most this many rays hand off at the floor from the start (see tail_policy)
   uint32_t skip_zero_terms;  // 1 (default traversal): shadow rays whose light term is exactly zero are answered without a walk
+};
+
+// slots of Levels::stats
+enum : uint32_t {
+  CRT_STAT_RAYS_PRIMARY = 0, CRT_STAT_RAYS_SHADOW = 1, CRT_STAT_RAYS_REFLECTION = 2, CRT_STAT_RAYS_REFRACTION = 3,
+  CRT_STAT_NODES_CLOSEST = 4, CRT_STAT_TRIS_CLOSEST = 5, CRT_STAT_NODES_SHADOW = 6, CRT_STAT_TRIS_SHADOW = 7,
+  CRT_STAT_PHASE = 8,       // CRT_PHASE_CLOCKS: 8 phase clocks / counts of k_closest, then 8 of k_shadow
+  CRT_STAT_WARP_SPAN = 24,  // CRT_PHASE_CLOCKS: warp lifetimes, warps, last end, first start of k_closest, then k_shadow
+  CRT_STAT_HANDOFF_CLOSEST = 32, CRT_STAT_HANDOFF_SHADOW = 33,  // walks handed to k_coop
+  CRT_STAT_COOP_DEBUG = 34,  // CRT_COOP_STATS: iterations, box tests, triangle tests of k_coop closest, then shadow
+  CRT_STAT_ZERO_TERM = 40,   // shadow rays answered without a walk
+  CRT_STAT_DIFFUSE = 41, CRT_STAT_PX_SAMPLES = 42, CRT_STAT_STOPPED = 43,
+  CRT_STAT_SLOTS = 48
 };
 
 // COMB_GI = {kind, first diffuse child (CRT_INVALID: beyond max_depth, every child is the background), diffuse item, G}
@@ -151,7 +164,7 @@ CRT_DI uint32_t level0_items(const Frame &fr) { return (LIST && fr.list) ? *fr.n
 //                (a lane has at most one pending leaf), so closest_offer sees exactly the sequence of KDTree.cpp:59-63.
 // ------------------------------------------------------------------------------------------------------------
 // CRT_PHASE_CLOCKS (debug builds for tools/ only): per-warp clock64 time spent in the refill / between-trees / node /
-// triangle phases of the MODE 2 kernels, plus iteration counts, summed into stats[8 + 8 * kernel + i] and printed by
+// triangle phases of the MODE 2 kernels, plus iteration counts, summed into stats[CRT_STAT_PHASE + 8 * kernel + i] and printed by
 // crtb200_core.cu after every frame.
 #ifndef CRT_PHASE_CLOCKS
 #define CRT_PHASE_CLOCKS 0
@@ -174,11 +187,11 @@ __device__ unsigned long long g_iter_hist[2][32];  // debug: rays by floor(log2(
 #define CRT_PC_MARK(i) { const long long n_ = clock64(); pc_acc[i] += (unsigned long long)(n_ - pc_t); pc_t = n_; }
 #define CRT_PC_COUNT(i, v) { pc_acc[i] += (v); }
 #define CRT_PC_FLUSH(base) { if (lane_id() == 0) { for (int i_ = 0; i_ < 8; i_++) atomicAdd(&lv.stats[(base) + i_], pc_acc[i_]); \
-    const unsigned long long g1_ = crt_globaltimer(); const int kb_ = 24 + ((base) - 8) / 2; /* 24.. closest, 28.. shadow */ \
+    const unsigned long long g1_ = crt_globaltimer(); const int kb_ = CRT_STAT_WARP_SPAN + ((base) - CRT_STAT_PHASE) / 2; \
     atomicAdd(&lv.stats[kb_], g1_ - pc_g0); atomicAdd(&lv.stats[kb_ + 1], 1ull); atomicMax(&lv.stats[kb_ + 2], g1_); \
     atomicMin(&lv.stats[kb_ + 3], pc_g0 ? pc_g0 : 1ull); \
-    atomicAdd(&g_tail[((base) - 8) / 8][0], pc_tail_time); atomicAdd(&g_tail[((base) - 8) / 8][1], pc_tail_lanes); \
-    const uint32_t w_ = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; if (w_ < 8192u) { unsigned long long *r_ = g_warp_rec[((base) - 8) / 8][w_]; \
+    atomicAdd(&g_tail[((base) - CRT_STAT_PHASE) / 8][0], pc_tail_time); atomicAdd(&g_tail[((base) - CRT_STAT_PHASE) / 8][1], pc_tail_lanes); \
+    const uint32_t w_ = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; if (w_ < 8192u) { unsigned long long *r_ = g_warp_rec[((base) - CRT_STAT_PHASE) / 8][w_]; \
       r_[0] = pc_g0; r_[1] = g1_; r_[2] = pc_acc[7]; r_[3] = pc_acc[5]; r_[4] = pc_tail_time; r_[5] = pc_acc[6]; } } }
 #else
 #define CRT_PC_TAIL(exh, act)
@@ -505,7 +518,7 @@ __global__ void __launch_bounds__(CRT_TRAV_BLOCK, PRIMARY ? CRT_TRAV_MIN_BLOCKS 
       CRT_PC_MARK(3)
     }
   }
-  CRT_PC_FLUSH(8)
+  CRT_PC_FLUSH(CRT_STAT_PHASE)
   if (COUNT) {
     unsigned long long a = n_nodes, b = n_tris;
 #pragma unroll
@@ -514,8 +527,8 @@ __global__ void __launch_bounds__(CRT_TRAV_BLOCK, PRIMARY ? CRT_TRAV_MIN_BLOCKS 
       b += __shfl_xor_sync(CRT_FULL_MASK, b, d);
     }
     if (lane == 0) {
-      atomicAdd(&lv.stats[4], a);
-      atomicAdd(&lv.stats[5], b);
+      atomicAdd(&lv.stats[CRT_STAT_NODES_CLOSEST], a);
+      atomicAdd(&lv.stats[CRT_STAT_TRIS_CLOSEST], b);
     }
   }
 }
@@ -753,15 +766,15 @@ __global__ void __launch_bounds__(256) k_shade(const DScene sc, const Frame fr, 
     c += __shfl_xor_sync(CRT_FULL_MASK, c, s);
   }
   if (lane_id() == 0) {
-    if (a) atomicAdd(&lv.stats[0], a);
-    if (b) atomicAdd(&lv.stats[2], b);
-    if (c) atomicAdd(&lv.stats[3], c);
+    if (a) atomicAdd(&lv.stats[CRT_STAT_RAYS_PRIMARY], a);
+    if (b) atomicAdd(&lv.stats[CRT_STAT_RAYS_REFLECTION], b);
+    if (c) atomicAdd(&lv.stats[CRT_STAT_RAYS_REFRACTION], c);
   }
   if (GI) {
     unsigned long long g = n_diff;
 #pragma unroll
     for (int s = 16; s > 0; s >>= 1) g += __shfl_xor_sync(CRT_FULL_MASK, g, s);
-    if (lane_id() == 0 && g) atomicAdd(&lv.stats[41], g);
+    if (lane_id() == 0 && g) atomicAdd(&lv.stats[CRT_STAT_DIFFUSE], g);
   }
 }
 
@@ -925,12 +938,12 @@ __global__ void __launch_bounds__(CRT_TRAV_BLOCK, CRT_TRAV_MIN_BLOCKS) k_shadow(
       CRT_PC_MARK(3)
     }
   }
-  CRT_PC_FLUSH(16)
+  CRT_PC_FLUSH(CRT_STAT_PHASE + 8)
   {
     uint32_t m = n_moot;
 #pragma unroll
     for (int d = 16; d > 0; d >>= 1) m += __shfl_xor_sync(CRT_FULL_MASK, m, d);
-    if (lane == 0 && m) atomicAdd(&lv.stats[40], (unsigned long long)m);
+    if (lane == 0 && m) atomicAdd(&lv.stats[CRT_STAT_ZERO_TERM], (unsigned long long)m);
   }
   if (COUNT) {
     unsigned long long a = n_nodes, b = n_tris;
@@ -940,8 +953,8 @@ __global__ void __launch_bounds__(CRT_TRAV_BLOCK, CRT_TRAV_MIN_BLOCKS) k_shadow(
       b += __shfl_xor_sync(CRT_FULL_MASK, b, d);
     }
     if (lane == 0) {
-      atomicAdd(&lv.stats[6], a);
-      atomicAdd(&lv.stats[7], b);
+      atomicAdd(&lv.stats[CRT_STAT_NODES_SHADOW], a);
+      atomicAdd(&lv.stats[CRT_STAT_TRIS_SHADOW], b);
     }
   }
 }
@@ -985,7 +998,7 @@ __global__ void __launch_bounds__(CRT_TRAV_BLOCK, CRT_TRAV_MIN_BLOCKS) k_shadow(
 #define CRT_COOP_MIN_BLOCKS 6  // resident CTAs per SM the register allocation is bounded for (24 warps = 96 walks per SM)
 #endif
 #ifndef CRT_COOP_STATS
-#define CRT_COOP_STATS 0  // debug builds (tools/): iterations, box tests and triangle tests of k_coop into stats[34..39]
+#define CRT_COOP_STATS 0  // debug builds (tools/): iterations, box tests and triangle tests of k_coop into stats[CRT_STAT_COOP_DEBUG ..]
 #endif
 #ifndef CRT_COOP_GROUP
 #define CRT_COOP_GROUP 32   // lanes per walk (8 and 16 measured: same throughput, longer walks; profiles/r2_tuning.md)
@@ -1073,7 +1086,7 @@ __global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_co
   // the GPU against the kernel it waits for.  early = 0: launched behind both; takes whatever is still published.
   volatile uint32_t *const ctl = lv.ovf_ctl + CRT_CTL_STRIDE * launch;
   const uint32_t n_rec = early ? lv.ovf_cap : min(ctl[0], lv.ovf_cap);
-  if (!early && blockIdx.x == 0 && threadIdx.x == 0 && n_rec) atomicAdd(&lv.stats[SHADOW ? 33 : 32], (unsigned long long)n_rec);
+  if (!early && blockIdx.x == 0 && threadIdx.x == 0 && n_rec) atomicAdd(&lv.stats[SHADOW ? CRT_STAT_HANDOFF_SHADOW : CRT_STAT_HANDOFF_CLOSEST], (unsigned long long)n_rec);
 
   // group state: identical in all lanes of a group, except cb (per-lane partial results)
   bool busy = false, drained = false, in_mesh = false, occluded = false;
@@ -1348,9 +1361,9 @@ __global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_co
     }
   }
 #if CRT_COOP_STATS
-  atomicAdd(&lv.stats[SHADOW ? 37 : 34], dbg_iters);
-  atomicAdd(&lv.stats[SHADOW ? 38 : 35], dbg_nodes);
-  atomicAdd(&lv.stats[SHADOW ? 39 : 36], dbg_tris);
+  atomicAdd(&lv.stats[CRT_STAT_COOP_DEBUG + (SHADOW ? 3 : 0)], dbg_iters);
+  atomicAdd(&lv.stats[CRT_STAT_COOP_DEBUG + (SHADOW ? 4 : 1)], dbg_nodes);
+  atomicAdd(&lv.stats[CRT_STAT_COOP_DEBUG + (SHADOW ? 5 : 2)], dbg_tris);
 #endif
 }
 
@@ -1427,7 +1440,7 @@ __global__ void __launch_bounds__(256) k_resolve(const DScene sc, const Frame fr
 __global__ void __launch_bounds__(256) k_sample_acc(const DScene sc, const Frame fr, const Levels lv, float4 *__restrict__ acc,
                                                     uint2 *__restrict__ hit0) {
   if (blockIdx.x == 0 && threadIdx.x == 0 && fr.sample + 1u < fr.spp)
-    atomicAdd(&lv.stats[1], (unsigned long long)lv.counts[CRT_MAX_LEVELS] * sc.n_lights);
+    atomicAdd(&lv.stats[CRT_STAT_RAYS_SHADOW], (unsigned long long)lv.counts[CRT_MAX_LEVELS] * sc.n_lights);
   const bool last = fr.sample + 1u == fr.spp;
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x) {
     const uint32_t node = lv.offset[0] + i;
@@ -1550,7 +1563,7 @@ __global__ void __launch_bounds__(256) k_store(const DScene sc, const Frame fr, 
                                               float *__restrict__ slab) {
   // shadow rays traced for this chunk = diffuse hits x lights (one per pair even when cos = 0, RayTracer.cpp:314-317)
   if (blockIdx.x == 0 && threadIdx.x == 0)
-    atomicAdd(&lv.stats[1], (unsigned long long)lv.counts[CRT_MAX_LEVELS] * sc.n_lights);
+    atomicAdd(&lv.stats[CRT_STAT_RAYS_SHADOW], (unsigned long long)lv.counts[CRT_MAX_LEVELS] * sc.n_lights);
   store_items(
       sc, fr, rgb, rgb8, hits, slab, [&](uint32_t i) { return lv.color[lv.offset[0] + i]; },
       [&](uint32_t i) {
@@ -1596,7 +1609,7 @@ CRT_DI bool accum_sample(const Frame &fr, const Levels &lv, uint32_t node, uint3
 // shadow rays of every pass.
 __global__ void __launch_bounds__(256) k_accum_step(const DScene sc, const Frame fr, const Levels lv, float4 *__restrict__ sum,
                                                    float4 *__restrict__ sumsq, uint2 *__restrict__ hit0) {
-  if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&lv.stats[1], (unsigned long long)lv.counts[CRT_MAX_LEVELS] * sc.n_lights);
+  if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&lv.stats[CRT_STAT_RAYS_SHADOW], (unsigned long long)lv.counts[CRT_MAX_LEVELS] * sc.n_lights);
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < fr.n_items0; i += gridDim.x * blockDim.x)
     accum_sample<false>(fr, lv, lv.offset[0] + i, fr.item_begin + i, AdaptParams{}, sum, sumsq, hit0);
 }
@@ -1745,21 +1758,21 @@ __global__ void __launch_bounds__(256) k_adapt_compact(const Frame fr, const flo
 }
 
 // One adaptive pass, in place of k_accum_step: accum_sample with the stop rule at shard item list[j].  Counts the
-// pass's shadow rays as k_accum_step does, its pixel-samples into stats[42] and the pixels it stopped into stats[43].
+// pass's shadow rays as k_accum_step does, its pixel-samples into stats[CRT_STAT_PX_SAMPLES] and the pixels it stopped into stats[CRT_STAT_STOPPED].
 __global__ void __launch_bounds__(256) k_adapt_step(const DScene sc, const Frame fr, const Levels lv, const AdaptParams ap,
                                                    float4 *__restrict__ sum, float4 *__restrict__ sumsq,
                                                    uint2 *__restrict__ hit0) {
   const uint32_t n_act = *fr.n_list;
   if (blockIdx.x == 0 && threadIdx.x == 0) {
-    atomicAdd(&lv.stats[1], (unsigned long long)lv.counts[CRT_MAX_LEVELS] * sc.n_lights);
-    atomicAdd(&lv.stats[42], (unsigned long long)n_act);
+    atomicAdd(&lv.stats[CRT_STAT_RAYS_SHADOW], (unsigned long long)lv.counts[CRT_MAX_LEVELS] * sc.n_lights);
+    atomicAdd(&lv.stats[CRT_STAT_PX_SAMPLES], (unsigned long long)n_act);
   }
   const uint32_t stride = gridDim.x * blockDim.x;
   for (uint32_t base = blockIdx.x * blockDim.x + (threadIdx.x & ~31u); base < n_act; base += stride) {
     const uint32_t j = base + lane_id();
     const bool stop = j < n_act && accum_sample<true>(fr, lv, lv.offset[0] + j, fr.list[j], ap, sum, sumsq, hit0);
     const uint32_t stopped = __popc(__ballot_sync(CRT_FULL_MASK, stop));
-    if (lane_id() == 0 && stopped) atomicAdd(&lv.stats[43], (unsigned long long)stopped);
+    if (lane_id() == 0 && stopped) atomicAdd(&lv.stats[CRT_STAT_STOPPED], (unsigned long long)stopped);
   }
 }
 

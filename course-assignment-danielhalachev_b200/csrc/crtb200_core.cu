@@ -10,6 +10,8 @@
 #include <memory>
 #include <mutex>
 #include <thread>
+#include <type_traits>
+#include <utility>
 #include <cstdio>
 #include <cstdlib>
 #include <cmath>
@@ -129,13 +131,16 @@ struct DevBuf {
   }
 };
 
+// counters of a render kept beside crtb200_stats: diffuse rays, and an adaptive step's pixel-samples and stopped pixels
+struct SideCounts { uint64_t diffuse = 0, px_samples = 0, stopped = 0; };
+
 struct crtb200_ctx {
   int device = 0;
   int sm_count = 0;
   cudaStream_t stream = nullptr;
-  cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
+  cudaEvent_t ev[2] = {nullptr, nullptr};  // the last frame's span on the caller's stream
   std::vector<cudaEvent_t> kev;  // per-launch event pairs: K2 / K3 timing
-  std::vector<int> kev_kind;     // 0 = closest, 1 = shadow (one entry per pair)
+  std::vector<int> kev_kind;     // 0 = closest, 1 = shadow, 2 / 3 their k_coop part (one entry per pair)
   size_t kev_used = 0;
   bool have_scene = false;
   uint64_t queue_budget = 16ull << 30;
@@ -246,10 +251,11 @@ struct crtb200_ctx {
   int blocks_closest = 0, blocks_closest_sec = 0, blocks_shadow = 0, blocks_coop = 0;
   crtb200_stats last{};
   bool last_pending = false;
+  bool bands_copied = false;  // the last enqueue_frame copied its host destinations band by band
   // sampling contract (crtb200_set_sampling); sampling.use_gi = 0: unsampled frames
   crtb200_sampling sampling{};
   uint32_t frame_offset = 0;  // crtb200_render_frames: added to sampling.frame_index for frame f
-  uint64_t last_diffuse = 0;  // diffuse rays of the last render (stats[41])
+  SideCounts last_side;
   uint32_t last_samples = 1;
   uint32_t cap_branch = 0;    // worst-case children per ray-tree node the queues were planned for
   uint32_t n_triangles = 0;   // of the uploaded scene (crtb200_accum_load checks the hit records it is given)
@@ -269,7 +275,6 @@ struct crtb200_ctx {
   bool acc_adaptive = false;
   AdaptParams acc_ap{};
   uint64_t acc_covered = 0, acc_active_px = 0, acc_px_samples = 0;
-  uint64_t last_px_samples = 0, last_stopped = 0;  // of the last adaptive step (stats[42], stats[43])
 
   // multi-GPU (crtb200_create_multi): this context is the primary (device_ids[0]).  A frame's 8x4-pixel tiles are dealt
   // round-robin over primary + peers (scene replicated); every GPU's k_store writes its pixels STRAIGHT into the
@@ -482,7 +487,7 @@ int crtb200_last_sampling_stats(crtb200_ctx *c, crtb200_sampling_stats *stats) {
   crtb200_stats unused;
   const int rc = crtb200_last_stats(c, &unused);  // synchronises a pending render_device frame
   if (rc) return rc;
-  stats->rays_diffuse = c->last_diffuse;
+  stats->rays_diffuse = c->last_side.diffuse;
   stats->samples = c->last_samples;
   stats->reserved = 0;
   return CRTB200_OK;
@@ -650,6 +655,13 @@ static float mesh_cull_margin(const crtb200_scene *s, const crtb200_mesh &me, bo
 
 static int upload_one(crtb200_ctx *c, const crtb200_scene *s);
 
+// the context and its peers, primary first: GPU i renders tile shard i
+static std::vector<crtb200_ctx *> all_gpus(crtb200_ctx *c) {
+  std::vector<crtb200_ctx *> gpus{c};
+  gpus.insert(gpus.end(), c->peers.begin(), c->peers.end());
+  return gpus;
+}
+
 // ends the progressive session of a context and frees its accumulators on every GPU
 static void accum_release(crtb200_ctx *c) {
   c->acc_active = false;
@@ -657,8 +669,7 @@ static void accum_release(crtb200_ctx *c) {
   c->acc_done = 0;
   c->acc_covered = c->acc_active_px = c->acc_px_samples = 0;
   c->acc_rects.clear();
-  for (size_t i = 0; i <= c->peers.size(); i++) {
-    crtb200_ctx *x = i ? c->peers[i - 1] : c;
+  for (crtb200_ctx *x : all_gpus(c)) {
     cudaSetDevice(x->device);
     x->acc_sum.release();
     x->acc_sumsq.release();
@@ -886,7 +897,7 @@ static int commit_scene(crtb200_ctx *c, const crtb200_scene *s, const SceneRecor
   CUDA_TRY(cudaMemset(c->frame.p, 0, px * 3 * sizeof(float)));  // colorBuffer starts at (0,0,0), RayTracer.cpp:47-50
   CUDA_TRY(c->frame8.ensure(px * 3));
   CUDA_TRY(cudaMemset(c->frame8.p, 0, px * 3));
-  CUDA_TRY(c->stats_dev.ensure(48));
+  CUDA_TRY(c->stats_dev.ensure(CRT_STAT_SLOTS));
   c->mask_valid = false;
   c->cap_items = 0;
   c->have_scene = true;
@@ -1445,81 +1456,100 @@ static cudaEvent_t next_event(crtb200_ctx *c) {
 // dynamic shared memory of the kernels that walk one ray per lane: the visited-mesh bitset of scenes with > 64 meshes
 static size_t dyn_smem(const crtb200_ctx *c, int block) { return (size_t)c->sc.dedup_words * (size_t)block * sizeof(uint32_t); }
 
-template <bool COUNT, bool CULL, bool WIDE>
-static void launch_closest_w(crtb200_ctx *c, bool primary, const Frame &fr, const Levels &lv, uint32_t level, uint32_t *work,
-                             cudaStream_t st) {
-  if (primary && fr.gi)
-    k_closest<true, COUNT, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, CULL, WIDE, true><<<c->blocks_closest, CRT_TRAV_BLOCK, dyn_smem(c, CRT_TRAV_BLOCK), st>>>(c->sc, fr, lv, level, work);
-  else if (primary)
-    k_closest<true, COUNT, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, CULL, WIDE><<<c->blocks_closest, CRT_TRAV_BLOCK, dyn_smem(c, CRT_TRAV_BLOCK), st>>>(c->sc, fr, lv, level, work);
-  else
-    k_closest<false, COUNT, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, CULL, WIDE><<<c->blocks_closest_sec, CRT_TRAV_BLOCK, dyn_smem(c, CRT_TRAV_BLOCK), st>>>(c->sc, fr, lv, level, work);
-}
-// the WIDE flavour (visited-mesh set in shared memory) only for scenes that need it, and never when counting the
-// reference's visit-all work (no de-duplication there)
-template <bool COUNT, bool CULL>
-static void launch_closest(crtb200_ctx *c, bool primary, const Frame &fr, const Levels &lv, uint32_t level, uint32_t *work,
-                           cudaStream_t st) {
-  if (!COUNT && c->sc.dedup_meshes == 2u)
-    launch_closest_w<COUNT, CULL, !COUNT>(c, primary, fr, lv, level, work, st);
-  else
-    launch_closest_w<COUNT, CULL, false>(c, primary, fr, lv, level, work, st);
-}
-template <int COUNT, bool CULL, bool SKIPR = true>
-static void launch_shadow(crtb200_ctx *c, const Frame &fr, const Levels &lv, uint32_t *work, cudaStream_t st) {
-  if (COUNT != 1 && c->sc.dedup_meshes == 2u)
-    k_shadow<COUNT, CRT_REFILL_SHADOW, CRT_LOOP_MODE, CULL, (COUNT != 1), SKIPR><<<c->blocks_shadow, CRT_TRAV_BLOCK, dyn_smem(c, CRT_TRAV_BLOCK), st>>>(c->sc, fr, lv, work);
-  else
-    k_shadow<COUNT, CRT_REFILL_SHADOW, CRT_LOOP_MODE, CULL, false, SKIPR><<<c->blocks_shadow, CRT_TRAV_BLOCK, 0, st>>>(c->sc, fr, lv, work);
-}
-// the shadow pass of one chunk in the flavour the options ask for; SKIPR = false in GI frames
-template <bool SKIPR>
-static void launch_shadow_pass(crtb200_ctx *c, const crtb200_options *o, bool cull, const Frame &fr, const Levels &lv, uint32_t *work,
-                               cudaStream_t st) {
-  if (o->count_work == 1)
-    launch_shadow<1, false, SKIPR>(c, fr, lv, work, st);
-  else if (o->count_work == 2 && cull)
-    launch_shadow<2, true, SKIPR>(c, fr, lv, work, st);
-  else if (o->count_work == 2)
-    launch_shadow<2, false, SKIPR>(c, fr, lv, work, st);
-  else if (cull)
-    launch_shadow<0, true, SKIPR>(c, fr, lv, work, st);
-  else
-    launch_shadow<0, false, SKIPR>(c, fr, lv, work, st);
+// The kernel flavours of one frame.  traversal 0 (default): conservative culling + tail hand-off, both exact and both
+// resting on the nesting property of the uploaded trees; traversal 1 and the visit-all counting mode walk the
+// reference's literal itinerary.  The WIDE flavour (visited-mesh set in shared memory) only for scenes that need it, and
+// never when counting the reference's visit-all work (no de-duplication there).
+struct Flavour {
+  uint32_t count_work;
+  bool cull, handoff, gi, wide_closest, wide_shadow;
+};
+
+static Flavour frame_flavour(const crtb200_ctx *c, const crtb200_options *o) {
+  const bool wide = c->sc.dedup_meshes == 2u;
+  return Flavour{o->count_work,
+                 o->traversal == 0 && o->count_work != 1 && c->nested_ok,
+                 o->traversal == 0 && o->count_work == 0 && c->nested_ok && c->tail_iters >= 0,
+                 c->sampling.use_gi != 0,
+                 o->count_work == 0 && wide,
+                 o->count_work != 1 && wide};
 }
 
-// k_coop around one traversal launch (DESIGN.md 3.8).  coop_begin forks the side stream BEFORE the traversal kernel is
-// launched; coop_end marks the traversal kernel's end behind it, starts the early pass on the side stream (its blocks
-// get SM resources as the traversal kernel's blocks exit), joins, and runs the final pass over what is left.
-static bool coop_early_on(const crtb200_ctx *c, bool secondary_level) {
-  return c->coop_early > 0 && c->cap_sets == 1 && !secondary_level;
+// f(v) with v as a compile-time constant: how the launch functions below turn a Flavour into template arguments
+template <typename F>
+static void as_const(bool v, F &&f) { v ? f(std::true_type{}) : f(std::false_type{}); }
+template <typename F>
+static void as_const_count(uint32_t v, F &&f) {
+  v == 1 ? f(std::integral_constant<int, 1>{}) : v == 2 ? f(std::integral_constant<int, 2>{}) : f(std::integral_constant<int, 0>{});
 }
-static int coop_begin(crtb200_ctx *c, crtb200_ctx::QueueSet &q, bool secondary_level) {
-  if (!coop_early_on(c, secondary_level)) return CRTB200_OK;
-  CUDA_TRY(cudaEventRecord(q.coop_fork, q.stream));
-  CUDA_TRY(cudaStreamWaitEvent(q.coop_stream, q.coop_fork, 0));
-  return CRTB200_OK;
+
+// k_closest of level `level`: PRIMARY at level 0, jittered in GI frames
+static void launch_closest(crtb200_ctx *c, const Flavour &fl, const Frame &fr, crtb200_ctx::QueueSet &q, uint32_t level) {
+  const bool primary = level == 0;
+  as_const(fl.count_work != 0, [&](auto count) { as_const(fl.cull, [&](auto cull) { as_const(fl.wide_closest, [&](auto wide) {
+    as_const(primary, [&](auto prim) { as_const(primary && fl.gi, [&](auto jitter) {
+      if constexpr (!(count && wide) && (prim || !jitter))
+        k_closest<prim, count, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, cull, wide, jitter>
+            <<<primary ? c->blocks_closest : c->blocks_closest_sec, CRT_TRAV_BLOCK, dyn_smem(c, CRT_TRAV_BLOCK), q.stream>>>(
+                c->sc, fr, q.lv, level, q.work + CRT_CTL_STRIDE * level);
+    }); }); }); }); });
 }
-template <bool SHADOW, bool CULL, bool SKIPR = true>
-static int coop_end(crtb200_ctx *c, crtb200_ctx::QueueSet &q, bool primary, const Frame &fr, uint32_t level, uint32_t &launches) {
-  const uint32_t launch = SHADOW ? (uint32_t)CRT_MAX_LEVELS : level;
-  auto run = [&](int blocks, cudaStream_t st, uint32_t early) {
-    if (SHADOW)
-      k_coop<true, false, CULL, CRT_COOP_GROUP, SKIPR><<<blocks, 32 * CRT_COOP_WARPS, 0, st>>>(c->sc, fr, q.lv, 0, early);
-    else if (primary)
-      k_coop<false, true, CULL, CRT_COOP_GROUP><<<blocks, 32 * CRT_COOP_WARPS, 0, st>>>(c->sc, fr, q.lv, level, early);
-    else
-      k_coop<false, false, CULL, CRT_COOP_GROUP><<<blocks, 32 * CRT_COOP_WARPS, 0, st>>>(c->sc, fr, q.lv, level, early);
-    launches++;
+// the shadow pass of one chunk; SKIPR = false in GI frames
+static void launch_shadow(crtb200_ctx *c, const Flavour &fl, const Frame &fr, crtb200_ctx::QueueSet &q) {
+  as_const_count(fl.count_work, [&](auto count) { as_const(fl.cull, [&](auto cull) { as_const(fl.wide_shadow, [&](auto wide) {
+    as_const(!fl.gi, [&](auto skipr) {
+      if constexpr (count != 1 || !(cull || wide))
+        k_shadow<count, CRT_REFILL_SHADOW, CRT_LOOP_MODE, cull, wide, skipr>
+            <<<c->blocks_shadow, CRT_TRAV_BLOCK, wide ? dyn_smem(c, CRT_TRAV_BLOCK) : 0, q.stream>>>(
+                c->sc, fr, q.lv, q.work + CRT_CTL_STRIDE * CRT_MAX_LEVELS);
+    }); }); }); });
+}
+// k_coop over the walks the shadow pass or closest-hit level `level` handed off; SKIPR = false in GI shadow passes
+static void launch_coop(crtb200_ctx *c, const Flavour &fl, const Frame &fr, crtb200_ctx::QueueSet &q, bool shadow, uint32_t level,
+                        int blocks, cudaStream_t st, uint32_t early) {
+  as_const(shadow, [&](auto sh) { as_const(!shadow && level == 0, [&](auto prim) { as_const(fl.cull, [&](auto cull) {
+    as_const(!(shadow && fl.gi), [&](auto skipr) {
+      if constexpr (!(sh && prim) && (sh || skipr))
+        k_coop<sh, prim, cull, CRT_COOP_GROUP, skipr><<<blocks, 32 * CRT_COOP_WARPS, 0, st>>>(c->sc, fr, q.lv, level, early);
+    }); }); }); });
+}
+
+// One traversal launch -- k_closest of level `level`, or the shadow pass -- and with hand-off k_coop around it (DESIGN.md
+// 3.8).  With an early pass (one queue set, not on a secondary level) the side stream is forked BEFORE the traversal
+// kernel is launched; behind it k_mark marks the traversal kernel's end, the early pass starts on the side stream (its
+// blocks get SM resources as the traversal kernel's blocks exit) and joins, and the final pass runs over what is left.
+// per_kernel: time them (closest_ms, shadow_ms, coop_*_ms); a mark with a kind (0 closest, 1 shadow, 2 / 3 their k_coop
+// part) opens a span and the next mark closes it, collect_stats_one reads them in pairs.
+static int traverse(crtb200_ctx *c, const Flavour &fl, const Frame &fr, crtb200_ctx::QueueSet &q, bool shadow, uint32_t level,
+                    bool per_kernel, uint32_t &launches) {
+  auto mark = [&](int kind) {
+    if (per_kernel) cudaEventRecord(next_event(c), q.stream);
+    if (per_kernel && kind >= 0) c->kev_kind.push_back(kind);
   };
-  if (coop_early_on(c, !SHADOW && !primary)) {
-    k_mark<<<1, 32, 0, q.stream>>>(q.lv.ovf_ctl + CRT_CTL_STRIDE * launch + 24u);
-    run(c->sm_count * c->coop_early, q.coop_stream, 1u);
-    CUDA_TRY(cudaEventRecord(q.coop_join, q.coop_stream));
-    CUDA_TRY(cudaStreamWaitEvent(q.stream, q.coop_join, 0));
+  const bool early = fl.handoff && c->coop_early > 0 && c->cap_sets == 1 && (shadow || level == 0);
+  mark(shadow ? 1 : 0);
+  if (early) {
+    CUDA_TRY(cudaEventRecord(q.coop_fork, q.stream));
+    CUDA_TRY(cudaStreamWaitEvent(q.coop_stream, q.coop_fork, 0));
+  }
+  if (shadow)
+    launch_shadow(c, fl, fr, q);
+  else
+    launch_closest(c, fl, fr, q, level);
+  if (fl.handoff) {
+    mark(-1);
+    mark(shadow ? 3 : 2);
+    if (early) {
+      k_mark<<<1, 32, 0, q.stream>>>(q.lv.ovf_ctl + CRT_CTL_STRIDE * (shadow ? (uint32_t)CRT_MAX_LEVELS : level) + 24u);
+      launch_coop(c, fl, fr, q, shadow, level, c->sm_count * c->coop_early, q.coop_stream, 1u);
+      CUDA_TRY(cudaEventRecord(q.coop_join, q.coop_stream));
+      CUDA_TRY(cudaStreamWaitEvent(q.stream, q.coop_join, 0));
+      launches += 2;
+    }
+    launch_coop(c, fl, fr, q, shadow, level, c->blocks_coop, q.stream, 0u);
     launches++;
   }
-  run(c->blocks_coop, q.stream, 0u);
+  mark(-1);
   return CRTB200_OK;
 }
 
@@ -1539,43 +1569,136 @@ struct AccumPass {
   const AdaptParams *ap;
 };
 
+// What a frame renders and where its pixels go; callers set the fields they use.
+struct FrameReq {
+  FrameReq(const crtb200_camera *cam, const crtb200_options *o) : cam(cam), o(o) {}
+  const crtb200_camera *cam;
+  const crtb200_options *o;
+  float *d_rgb = nullptr;  // device destinations (any may be null)
+  uint8_t *d_rgb8 = nullptr;
+  HitRec *d_hits = nullptr;
+  float *d_slab = nullptr;          // a tile shard's compact slab (crtb200_render_device)
+  const HostOut *host = nullptr;    // crtb200_render: band copies where the frame allows them (ctx->bands_copied)
+  bool batch_continuation = false;  // a frame after the first of crtb200_render_frames
+  const AccumPass *acc = nullptr;   // a step of a progressive session
+};
+
 // level-0 work items of tile shard `index` of `count`: 8x4-pixel tiles dealt round-robin, 32 items each
 static uint32_t shard_item_count(const crtb200_ctx *c, uint32_t index, uint32_t count) {
   const uint32_t tiles = ((c->sc.width + 7) / 8) * ((c->sc.height + 3) / 4);
   return (tiles > index ? (tiles - index + count - 1) / count : 0) * 32u;
 }
 
-// Enqueue one frame on `st`.  d_rgb / d_rgb8 / d_hits / d_slab are device pointers (any may be null).
-static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_options *o, float *d_rgb,
-                         uint8_t *d_rgb8, HitRec *d_hits, float *d_slab, cudaStream_t st, bool timed,
-                         const HostOut *host = nullptr, bool *host_done = nullptr, bool batch_continuation = false,
-                         const AccumPass *acc = nullptr) {
+// a Frame over the 8x4-pixel tiles of tile shard `index` of `count`, with the mask of the last plan_mask
+static Frame frame_tiles(const crtb200_ctx *c, uint32_t index, uint32_t count) {
+  Frame fr{};
+  fr.tiles_x = (c->sc.width + 7) / 8;
+  fr.n_tiles = fr.tiles_x * ((c->sc.height + 3) / 4);
+  fr.shard_index = index;
+  fr.shard_count = count;
+  fr.mask = c->mask_needed ? c->mask.p : nullptr;
+  return fr;
+}
+
+// One sample pass of one chunk (sample fr.sample): the level loop, the shadow pass, k_accumulate, k_resolve and the
+// kernel that ends a sample of a GI frame or a progressive step
+static int sample_pass(crtb200_ctx *c, const FrameReq &r, const Flavour &fl, Frame &fr, crtb200_ctx::QueueSet &q, uint32_t levels,
+                       bool per_kernel, uint32_t &launches) {
+  const cudaStream_t qs = q.stream;
+  const int grid_simple = c->sm_count * 8;
+  const bool adapt_step = r.acc && r.acc->ap;
+  CUDA_TRY(cudaMemsetAsync(q.ctl.p, 0, q.ctl.n * sizeof(uint32_t), qs));
+  if (adapt_step) {
+    // level 0 of this pass runs over the pixels still sampling; the host keeps n_items0 as the bound
+    fr.list = fr.n_list = nullptr;
+    CUDA_TRY(cudaMemsetAsync(q.acount.p, 0, sizeof(uint32_t), qs));
+    k_adapt_compact<<<grid_simple, 256, 0, qs>>>(fr, c->acc_sumsq.p, q.alist.p, q.acount.p);
+    launches++;
+    fr.list = q.alist.p;
+    fr.n_list = q.acount.p;
+  }
+  q.lv.tail_iters = fl.handoff ? (uint32_t)(c->tail_iters + 1) : 0u;
+  q.lv.skip_zero_terms = (r.o->traversal == 0 && r.o->count_work != 1) ? 1u : 0u;
+  q.lv.tail_start = (uint32_t)c->tail_start;
+  q.lv.tail_start_closest = (uint32_t)c->tail_start_closest;
+  q.lv.tail_small = (uint32_t)c->tail_small;
+  for (uint32_t l = 0; l < levels; l++) {
+    const int rc = traverse(c, fl, fr, q, false, l, per_kernel, launches);
+    if (rc) return rc;
+    as_const(fl.gi, [&](auto gi) { k_shade<gi><<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, l); });
+    launches += 2;
+  }
+  const int rc = traverse(c, fl, fr, q, true, 0, per_kernel, launches);
+  if (rc) return rc;
+  k_accumulate<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv);
+  launches += 2;
+  // (GI frames resolve the last level too: its diffuse hits combine D with G background children)
+  for (uint32_t l = fl.gi ? levels : levels - 1; l-- > 0;) {
+    as_const(fl.gi, [&](auto gi) { k_resolve<gi><<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, l); });
+    launches++;
+  }
+  if (adapt_step)
+    k_adapt_step<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, *r.acc->ap, c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p);
+  else if (r.acc)
+    k_accum_step<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p);
+  else if (fl.gi)
+    k_sample_acc<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, q.acc.p, q.hit0.p);
+  if (r.acc || fl.gi) launches++;
+  return CRTB200_OK;
+}
+
+// the band of image rows that chunk `chunk` (level-0 items [begin, begin + n)) has stored, to the host destinations:
+// behind the chunk's stream qs, on the band stream when there is one
+static int copy_band(crtb200_ctx *c, const FrameReq &r, cudaStream_t qs, uint32_t chunk, uint32_t begin, uint32_t n,
+                     uint32_t row_items, bool band_stream) {
+  const uint32_t W = c->sc.width, H = c->sc.height;
+  const uint32_t row0 = (begin / row_items) * 4u;
+  const uint32_t row1 = std::min<uint32_t>(H, ((begin + n + row_items - 1) / row_items) * 4u);
+  const size_t off = (size_t)row0 * W, cnt = (size_t)(row1 - row0) * W;
+  cudaStream_t cs = qs;
+  if (band_stream) {
+    CUDA_TRY(cudaEventRecord(c->chunk_done[chunk], qs));
+    CUDA_TRY(cudaStreamWaitEvent(c->band_stream, c->chunk_done[chunk], 0));
+    cs = c->band_stream;
+  }
+  const HostOut &h = *r.host;
+  if (h.rgb) CUDA_TRY(cudaMemcpyAsync(h.rgb + off * 3, r.d_rgb + off * 3, cnt * 3 * sizeof(float), cudaMemcpyDeviceToHost, cs));
+  if (h.rgb8) CUDA_TRY(cudaMemcpyAsync(h.rgb8 + off * 3, r.d_rgb8 + off * 3, cnt * 3, cudaMemcpyDeviceToHost, cs));
+  if (h.hits) CUDA_TRY(cudaMemcpyAsync(h.hits + off, r.d_hits + off, cnt * sizeof(HitRec), cudaMemcpyDeviceToHost, cs));
+  if (getenv("CRT_CHUNK_TIMES")) {
+    while (c->dbg_ev.size() < 2 * (size_t)(chunk + 1)) {
+      cudaEvent_t e = nullptr;
+      CUDA_TRY(cudaEventCreate(&e));
+      c->dbg_ev.push_back(e);
+    }
+    CUDA_TRY(cudaEventRecord(c->dbg_ev[2 * chunk], qs));
+    CUDA_TRY(cudaEventRecord(c->dbg_ev[2 * chunk + 1], cs));
+    c->dbg_chunks = chunk + 1;
+  }
+  return CRTB200_OK;
+}
+
+// Enqueue one frame on `st`; c->bands_copied then says whether the frame's host destinations are copied already.
+static int enqueue_frame(crtb200_ctx *c, const FrameReq &r, cudaStream_t st) {
+  const crtb200_options *o = r.o;
+  const AccumPass *acc = r.acc;
   if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
   if (o->max_depth > 31) return fail(CRTB200_ERR_ARG, "max_depth > 31 is not supported");
   if (o->n_rects && !o->rects) return fail(CRTB200_ERR_ARG, "n_rects > 0 but rects is null");
   if (o->traversal > 1) return fail(CRTB200_ERR_ARG, "unknown traversal mode");
   if (o->count_work > 2) return fail(CRTB200_ERR_ARG, "unknown count_work mode");
-  // traversal 0 (default): conservative culling + tail hand-off, both exact and both resting on the nesting property of
-  // the uploaded trees; traversal 1 and the visit-all counting mode walk the reference's literal itinerary
-  const bool cull = o->traversal == 0 && o->count_work != 1 && c->nested_ok;
-  const bool handoff = o->traversal == 0 && o->count_work == 0 && c->nested_ok && c->tail_iters >= 0;
+  const Flavour fl = frame_flavour(c, o);
   const uint32_t shard_count = o->shard_count ? o->shard_count : 1;
   if (o->shard_index >= shard_count) return fail(CRTB200_ERR_ARG, "shard_index >= shard_count");
   int rc = plan_mask(c, o);
   if (rc) return rc;
-  const uint32_t W = c->sc.width, H = c->sc.height;
-  Frame fr{};
-  for (int k = 0; k < 3; k++) fr.cam.pos[k] = cam->position[k];
-  for (int k = 0; k < 9; k++) fr.cam.rot[k] = cam->rotation[k];
-  fr.tiles_x = (W + 7) / 8;
-  fr.n_tiles = fr.tiles_x * ((H + 3) / 4);
-  fr.shard_index = o->shard_index;
-  fr.shard_count = shard_count;
-  fr.mask = c->mask_needed ? c->mask.p : nullptr;
+  Frame fr = frame_tiles(c, o->shard_index, shard_count);
+  for (int k = 0; k < 3; k++) fr.cam.pos[k] = r.cam->position[k];
+  for (int k = 0; k < 9; k++) fr.cam.rot[k] = r.cam->rotation[k];
   fr.max_depth = o->max_depth;
-  // GI frames (sampling contract, DESIGN.md 3.10): spp sample-major passes per chunk, each the whole level loop below
-  const bool gi = c->sampling.use_gi != 0;
-  fr.resolve = (c->has_reflective || c->has_refractive || gi) ? 1u : 0u;
+  // GI frames (sampling contract, DESIGN.md 3.10): spp sample-major passes per chunk, each the whole level loop
+  const bool gi = fl.gi, secondary = c->has_reflective || c->has_refractive || gi;
+  fr.resolve = secondary ? 1u : 0u;
   fr.shadow_bias = o->shadow_bias;
   fr.reflection_bias = o->reflection_bias;
   fr.refraction_bias = o->refraction_bias;
@@ -1588,32 +1711,29 @@ static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb20
   const uint32_t shard_items = shard_item_count(c, o->shard_index, shard_count);
   // unsharded frames: chunks are whole rows of tiles, so a chunk owns a contiguous band of image rows
   const uint32_t row_items = (shard_count == 1) ? fr.tiles_x * 32u : 32u;
-  rc = plan_queues(c, std::max(shard_items, 32u), o->max_depth, row_items, host != nullptr);
+  rc = plan_queues(c, std::max(shard_items, 32u), o->max_depth, row_items, r.host != nullptr);
   if (rc) return rc;
-  const bool secondary = c->has_reflective || c->has_refractive || gi;
   const uint32_t levels = secondary ? o->max_depth + 1 : 1;
   c->last_samples = acc ? acc->n : fr.spp;
   const uint32_t s_begin = acc ? acc->s0 : 0u, s_end = acc ? acc->s0 + acc->n : fr.spp;
   // Band copies need chunks that own whole rows of tiles: with a small queue budget or a deep refractive scene a chunk
   // is smaller than a tile row, two chunks on different streams would then share a 4-row band and a band copy could
   // pick up the other chunk's stale pixels.  Then the caller copies the whole frame after the join instead.
-  const bool band_copies = host && shard_count == 1 && c->cap_items % row_items == 0;
-  if (host_done) *host_done = band_copies;
-  const int grid_simple = c->sm_count * 8;
+  const bool band_copies = r.host && shard_count == 1 && c->cap_items % row_items == 0;
+  c->bands_copied = band_copies;
 
   // frames after the first of a batch (crtb200_render_frames) keep accumulating into the same counters and time span
-  if (!batch_continuation) CUDA_TRY(cudaMemsetAsync(c->stats_dev.p, 0, 48 * sizeof(unsigned long long), st));
+  if (!r.batch_continuation) CUDA_TRY(cudaMemsetAsync(c->stats_dev.p, 0, CRT_STAT_SLOTS * sizeof(unsigned long long), st));
 #if CRT_PHASE_CLOCKS
-  CUDA_TRY(cudaMemsetAsync(c->stats_dev.p + 27, 0xFF, sizeof(unsigned long long), st));  // atomicMin slots
-  CUDA_TRY(cudaMemsetAsync(c->stats_dev.p + 31, 0xFF, sizeof(unsigned long long), st));
+  CUDA_TRY(cudaMemsetAsync(c->stats_dev.p + CRT_STAT_WARP_SPAN + 3, 0xFF, sizeof(unsigned long long), st));  // atomicMin slots
+  CUDA_TRY(cudaMemsetAsync(c->stats_dev.p + CRT_STAT_WARP_SPAN + 7, 0xFF, sizeof(unsigned long long), st));
 #endif
   c->kev_used = 0;
   c->kev_kind.clear();
-  if (timed && !batch_continuation) CUDA_TRY(cudaEventRecord(c->ev[0], st));
-  // fork: every set's stream waits for the caller's stream, chunks go round-robin, the caller's stream joins at the end.
-  // Per-kernel event pairs are only recorded without concurrency (overlapping kernels would inflate each other).
+  if (!r.batch_continuation) CUDA_TRY(cudaEventRecord(c->ev[0], st));
+  // fork: every set's stream waits for the caller's stream, chunks go round-robin, the caller's stream joins at the end
   const uint32_t n_sets = c->cap_sets;
-  const bool per_kernel = timed && n_sets == 1 && !batch_continuation;
+  const bool per_kernel = n_sets == 1 && !r.batch_continuation;
   CUDA_TRY(cudaEventRecord(c->fork_ev, st));
   for (uint32_t k = 0; k < n_sets; k++) CUDA_TRY(cudaStreamWaitEvent(c->sets[k].stream, c->fork_ev, 0));
   uint32_t launches = 0, chunk = 0;
@@ -1630,142 +1750,28 @@ static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb20
   }
   for (uint32_t begin = 0; begin < shard_items; begin += c->cap_items, chunk++) {
     crtb200_ctx::QueueSet &q = c->sets[chunk % n_sets];
-    cudaStream_t qs = q.stream;
     fr.item_begin = begin;
     fr.n_items0 = std::min(c->cap_items, shard_items - begin);
     if (gi && !acc) {
       CUDA_TRY(q.acc.ensure(c->cap_items));
       CUDA_TRY(q.hit0.ensure(c->cap_items));
     }
-    const bool adapt_step = acc && acc->ap;
-    if (adapt_step) {
+    if (acc && acc->ap) {
       CUDA_TRY(q.alist.ensure(c->cap_items));
       CUDA_TRY(q.acount.ensure(1));
     }
     for (uint32_t s = s_begin; s < s_end; s++) {
       fr.sample = s;
-      CUDA_TRY(cudaMemsetAsync(q.ctl.p, 0, q.ctl.n * sizeof(uint32_t), qs));
-      if (adapt_step) {
-        // level 0 of this pass runs over the pixels still sampling; the host keeps n_items0 as the bound
-        fr.list = fr.n_list = nullptr;
-        CUDA_TRY(cudaMemsetAsync(q.acount.p, 0, sizeof(uint32_t), qs));
-        k_adapt_compact<<<grid_simple, 256, 0, qs>>>(fr, c->acc_sumsq.p, q.alist.p, q.acount.p);
-        launches++;
-        fr.list = q.alist.p;
-        fr.n_list = q.acount.p;
-      }
-      q.lv.tail_iters = handoff ? (uint32_t)(c->tail_iters + 1) : 0u;
-      q.lv.skip_zero_terms = (o->traversal == 0 && o->count_work != 1) ? 1u : 0u;
-      q.lv.tail_start = (uint32_t)c->tail_start;
-      q.lv.tail_start_closest = (uint32_t)c->tail_start_closest;
-      q.lv.tail_small = (uint32_t)c->tail_small;
-      for (uint32_t l = 0; l < levels; l++) {
-        if (per_kernel) {
-          cudaEventRecord(next_event(c), qs);
-          c->kev_kind.push_back(0);
-        }
-        if (handoff) {
-          rc = coop_begin(c, q, l != 0);
-          if (rc) return rc;
-        }
-        if (o->count_work && cull)
-          launch_closest<true, true>(c, l == 0, fr, q.lv, l, q.work + CRT_CTL_STRIDE * l, qs);
-        else if (o->count_work)
-          launch_closest<true, false>(c, l == 0, fr, q.lv, l, q.work + CRT_CTL_STRIDE * l, qs);
-        else if (cull)
-          launch_closest<false, true>(c, l == 0, fr, q.lv, l, q.work + CRT_CTL_STRIDE * l, qs);
-        else
-          launch_closest<false, false>(c, l == 0, fr, q.lv, l, q.work + CRT_CTL_STRIDE * l, qs);
-        if (handoff) {
-          if (per_kernel) {
-            cudaEventRecord(next_event(c), qs);
-            cudaEventRecord(next_event(c), qs);
-            c->kev_kind.push_back(2);
-          }
-          rc = cull ? coop_end<false, true>(c, q, l == 0, fr, l, launches) : coop_end<false, false>(c, q, l == 0, fr, l, launches);
-          if (rc) return rc;
-        }
-        if (per_kernel) cudaEventRecord(next_event(c), qs);
-        if (gi)
-          k_shade<true><<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, l);
-        else
-          k_shade<false><<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, l);
-        launches += 2;
-      }
-      if (per_kernel) {
-        cudaEventRecord(next_event(c), qs);
-        c->kev_kind.push_back(1);
-      }
-      uint32_t *swork = q.work + CRT_CTL_STRIDE * CRT_MAX_LEVELS;
-      if (handoff) {
-        rc = coop_begin(c, q, false);
-        if (rc) return rc;
-      }
-      if (gi)
-        launch_shadow_pass<false>(c, o, cull, fr, q.lv, swork, qs);
-      else
-        launch_shadow_pass<true>(c, o, cull, fr, q.lv, swork, qs);
-      if (handoff) {
-        if (per_kernel) {
-          cudaEventRecord(next_event(c), qs);
-          cudaEventRecord(next_event(c), qs);
-          c->kev_kind.push_back(3);
-        }
-        if (gi)
-          rc = cull ? coop_end<true, true, false>(c, q, false, fr, 0, launches) : coop_end<true, false, false>(c, q, false, fr, 0, launches);
-        else
-          rc = cull ? coop_end<true, true>(c, q, false, fr, 0, launches) : coop_end<true, false>(c, q, false, fr, 0, launches);
-        if (rc) return rc;
-      }
-      if (per_kernel) cudaEventRecord(next_event(c), qs);
-      k_accumulate<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv);
-      launches += 2;
-      // (GI frames resolve the last level too: its diffuse hits combine D with G background children)
-      for (uint32_t l = gi ? levels : levels - 1; l-- > 0;) {
-        if (gi)
-          k_resolve<true><<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, l);
-        else
-          k_resolve<false><<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, l);
-        launches++;
-      }
-      if (adapt_step) {
-        k_adapt_step<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, *acc->ap, c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p);
-        launches++;
-      } else if (acc) {
-        k_accum_step<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p);
-        launches++;
-      } else if (gi) {
-        k_sample_acc<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, q.acc.p, q.hit0.p);
-        launches++;
-      }
+      rc = sample_pass(c, r, fl, fr, q, levels, per_kernel, launches);
+      if (rc) return rc;
     }
     if (!acc) {
-      k_store<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, d_rgb, d_rgb8, d_hits, d_slab);
+      k_store<<<c->sm_count * 8, 256, 0, q.stream>>>(c->sc, fr, q.lv, r.d_rgb, r.d_rgb8, r.d_hits, r.d_slab);
       launches++;
     }
     if (band_copies) {
-      const uint32_t row0 = (begin / row_items) * 4u;
-      const uint32_t row1 = std::min<uint32_t>(H, ((begin + fr.n_items0 + row_items - 1) / row_items) * 4u);
-      const size_t off = (size_t)row0 * W, cnt = (size_t)(row1 - row0) * W;
-      cudaStream_t cs = qs;
-      if (band_stream) {
-        CUDA_TRY(cudaEventRecord(c->chunk_done[chunk], qs));
-        CUDA_TRY(cudaStreamWaitEvent(c->band_stream, c->chunk_done[chunk], 0));
-        cs = c->band_stream;
-      }
-      if (host->rgb) CUDA_TRY(cudaMemcpyAsync(host->rgb + off * 3, d_rgb + off * 3, cnt * 3 * sizeof(float), cudaMemcpyDeviceToHost, cs));
-      if (host->rgb8) CUDA_TRY(cudaMemcpyAsync(host->rgb8 + off * 3, d_rgb8 + off * 3, cnt * 3, cudaMemcpyDeviceToHost, cs));
-      if (host->hits) CUDA_TRY(cudaMemcpyAsync(host->hits + off, d_hits + off, cnt * sizeof(HitRec), cudaMemcpyDeviceToHost, cs));
-      if (getenv("CRT_CHUNK_TIMES")) {
-        while (c->dbg_ev.size() < 2 * (size_t)(chunk + 1)) {
-          cudaEvent_t e = nullptr;
-          CUDA_TRY(cudaEventCreate(&e));
-          c->dbg_ev.push_back(e);
-        }
-        CUDA_TRY(cudaEventRecord(c->dbg_ev[2 * chunk], qs));
-        CUDA_TRY(cudaEventRecord(c->dbg_ev[2 * chunk + 1], cs));
-        c->dbg_chunks = chunk + 1;
-      }
+      rc = copy_band(c, r, q.stream, chunk, begin, fr.n_items0, row_items, band_stream);
+      if (rc) return rc;
     }
   }
   if (band_stream) {
@@ -1776,7 +1782,7 @@ static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb20
     CUDA_TRY(cudaEventRecord(c->sets[k].done, c->sets[k].stream));
     CUDA_TRY(cudaStreamWaitEvent(st, c->sets[k].done, 0));
   }
-  if (timed) CUDA_TRY(cudaEventRecord(c->ev[1], st));
+  CUDA_TRY(cudaEventRecord(c->ev[1], st));
   CUDA_TRY(cudaGetLastError());
   c->last.kernel_launches = launches;
   c->last.levels = levels;
@@ -1784,30 +1790,32 @@ static int enqueue_frame(crtb200_ctx *c, const crtb200_camera *cam, const crtb20
 }
 
 // Multi-GPU frame (crtb200_create_multi): shard i of n goes to GPU i; every GPU stores into the SAME destination
-// buffers (device memory of the primary, peer-mapped on the others).  The peers start after `st` has reached this point
-// (earlier consumers of the frame on the primary's stream are done) and `st` continues after every peer has stored.
-static int enqueue_any(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_options *o, float *d_rgb, uint8_t *d_rgb8,
-                       HitRec *d_hits, float *d_slab, cudaStream_t st, bool timed, const HostOut *host = nullptr,
-                       bool *host_done = nullptr, bool batch_continuation = false, const AccumPass *acc = nullptr) {
-  if (c->peers.empty() || o->shard_count > 1)
-    return enqueue_frame(c, cam, o, d_rgb, d_rgb8, d_hits, d_slab, st, timed, host, host_done, batch_continuation, acc);
-  if (host_done) *host_done = false;  // the caller copies the assembled frame after the join
+// buffers (device memory of the primary, peer-mapped on the others), and the caller copies the assembled frame to the
+// host after the join.  The peers start after `st` has reached this point (earlier consumers of the frame on the
+// primary's stream are done) and `st` continues after every peer has stored.
+static int enqueue_any(crtb200_ctx *c, const FrameReq &r, cudaStream_t st) {
+  if (c->peers.empty() || r.o->shard_count > 1) return enqueue_frame(c, r, st);
   const uint32_t n = 1u + (uint32_t)c->peers.size();
   CUDA_TRY(cudaSetDevice(c->device));
   CUDA_TRY(cudaEventRecord(c->multi_fork, st));
-  crtb200_options o0 = *o;
+  crtb200_options o0 = *r.o;
   o0.shard_index = 0;
   o0.shard_count = n;
+  FrameReq r0 = r;
+  r0.o = &o0;
+  r0.host = nullptr;
   int rc = on_all_devices(
-      c, [&] { return enqueue_frame(c, cam, &o0, d_rgb, d_rgb8, d_hits, nullptr, st, timed, nullptr, nullptr, batch_continuation, acc); },
+      c, [&] { return enqueue_frame(c, r0, st); },
       [&](size_t i, crtb200_ctx *p) {
-        crtb200_options oi = *o;
+        crtb200_options oi = *r.o;
         oi.shard_index = (uint32_t)i + 1u;
         oi.shard_count = n;
+        FrameReq ri = r0;
+        ri.o = &oi;
         CUDA_TRY(cudaSetDevice(p->device));
         CUDA_TRY(cudaStreamWaitEvent(p->stream, c->multi_fork, 0));
-        int r = enqueue_frame(p, cam, &oi, d_rgb, d_rgb8, d_hits, nullptr, p->stream, true, nullptr, nullptr, batch_continuation, acc);
-        if (r) return r;
+        int e = enqueue_frame(p, ri, p->stream);
+        if (e) return e;
         p->last_pending = true;
         CUDA_TRY(cudaEventRecord(p->multi_done, p->stream));
         return (int)CRTB200_OK;
@@ -1815,48 +1823,16 @@ static int enqueue_any(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_
   CUDA_TRY(cudaSetDevice(c->device));
   if (rc) return rc;
   for (crtb200_ctx *p : c->peers) CUDA_TRY(cudaStreamWaitEvent(st, p->multi_done, 0));
-  if (timed) CUDA_TRY(cudaEventRecord(c->ev[1], st));  // the frame ends when the last GPU has stored its shard
-  return CRTB200_OK;
-}
-
-static int collect_stats_one(crtb200_ctx *c, bool timed);
-// counters of the primary plus those of the peers (rays, tests, launches); times are the primary's (fork to join)
-static int collect_stats(crtb200_ctx *c, bool timed) {
-  int rc = collect_stats_one(c, timed);
-  if (rc) return rc;
-  for (crtb200_ctx *p : c->peers) {
-    if (!p->last_pending) continue;
-    CUDA_TRY(cudaSetDevice(p->device));
-    CUDA_TRY(cudaStreamSynchronize(p->stream));
-    rc = collect_stats_one(p, false);
-    p->last_pending = false;
-    if (rc) return rc;
-    c->last.rays_primary += p->last.rays_primary;
-    c->last.rays_shadow += p->last.rays_shadow;
-    c->last.rays_reflection += p->last.rays_reflection;
-    c->last.rays_refraction += p->last.rays_refraction;
-    c->last.node_tests_closest += p->last.node_tests_closest;
-    c->last.triangle_tests_closest += p->last.triangle_tests_closest;
-    c->last.node_tests_shadow += p->last.node_tests_shadow;
-    c->last.triangle_tests_shadow += p->last.triangle_tests_shadow;
-    c->last.handoff_closest += p->last.handoff_closest;
-    c->last.handoff_shadow += p->last.handoff_shadow;
-    c->last.shadow_rays_zero_term += p->last.shadow_rays_zero_term;
-    c->last.kernel_launches += p->last.kernel_launches;
-    c->last_diffuse += p->last_diffuse;
-    c->last_px_samples += p->last_px_samples;
-    c->last_stopped += p->last_stopped;
-  }
-  CUDA_TRY(cudaSetDevice(c->device));
+  CUDA_TRY(cudaEventRecord(c->ev[1], st));  // the frame ends when the last GPU has stored its shard
   return CRTB200_OK;
 }
 
 static int collect_stats_one(crtb200_ctx *c, bool timed) {
-  unsigned long long st[48];
+  unsigned long long st[CRT_STAT_SLOTS];
   CUDA_TRY(cudaMemcpy(st, c->stats_dev.p, sizeof(st), cudaMemcpyDeviceToHost));
 #if CRT_PHASE_CLOCKS
   for (int k = 0; k < 2; k++) {
-    const unsigned long long *p = st + 8 + 8 * k;
+    const unsigned long long *p = st + CRT_STAT_PHASE + 8 * k;
     const double tot = (double)(p[0] + p[1] + p[2] + p[3] + p[4]);
     fprintf(stderr, "[phase clocks] %s: refill %.1f%% slow %.1f%% node %.1f%% tri %.1f%% other %.1f%% | node iterations %llu, tri phases (MODE 2) / ranges stolen (k_*_s) %llu, rounds %llu\n",
             k ? "k_shadow " : "k_closest", 100.0 * p[0] / tot, 100.0 * p[1] / tot, 100.0 * p[2] / tot, 100.0 * p[3] / tot, 100.0 * p[4] / tot,
@@ -1892,29 +1868,28 @@ static int collect_stats_one(crtb200_ctx *c, bool timed) {
                 (r[0] - t0) * 1e-3, (r[1] - t0) * 1e-3, r[2], r[3], r[4], r[5]);
       }
     }
-    const unsigned long long *g = st + 24 + 4 * k;  // sum of warp lifetimes, warps, last end, first start (globaltimer ns)
+    const unsigned long long *g = st + CRT_STAT_WARP_SPAN + 4 * k;  // sum of warp lifetimes, warps, last end, first start (globaltimer ns)
     if (g[1])
       fprintf(stderr, "[phase clocks] %s: %llu warps, mean warp lifetime %.1f us, kernel span %.1f us (first warp start -> last warp end; one launch per frame only)\n",
               k ? "k_shadow " : "k_closest", g[1], 1e-3 * (double)g[0] / (double)g[1], 1e-3 * (double)(g[2] - g[3]));
   }
 #endif
-  c->last.rays_primary = st[0];
-  c->last.rays_shadow = st[1];
-  c->last.rays_reflection = st[2];
-  c->last.rays_refraction = st[3];
-  c->last.node_tests_closest = st[4];
-  c->last.triangle_tests_closest = st[5];
-  c->last.node_tests_shadow = st[6];
-  c->last.triangle_tests_shadow = st[7];
-  c->last.handoff_closest = st[32];
-  c->last.handoff_shadow = st[33];
-  c->last.shadow_rays_zero_term = st[40];
-  c->last_diffuse = st[41];
-  c->last_px_samples = st[42];
-  c->last_stopped = st[43];
+  c->last.rays_primary = st[CRT_STAT_RAYS_PRIMARY];
+  c->last.rays_shadow = st[CRT_STAT_RAYS_SHADOW];
+  c->last.rays_reflection = st[CRT_STAT_RAYS_REFLECTION];
+  c->last.rays_refraction = st[CRT_STAT_RAYS_REFRACTION];
+  c->last.node_tests_closest = st[CRT_STAT_NODES_CLOSEST];
+  c->last.triangle_tests_closest = st[CRT_STAT_TRIS_CLOSEST];
+  c->last.node_tests_shadow = st[CRT_STAT_NODES_SHADOW];
+  c->last.triangle_tests_shadow = st[CRT_STAT_TRIS_SHADOW];
+  c->last.handoff_closest = st[CRT_STAT_HANDOFF_CLOSEST];
+  c->last.handoff_shadow = st[CRT_STAT_HANDOFF_SHADOW];
+  c->last.shadow_rays_zero_term = st[CRT_STAT_ZERO_TERM];
+  c->last_side = SideCounts{st[CRT_STAT_DIFFUSE], st[CRT_STAT_PX_SAMPLES], st[CRT_STAT_STOPPED]};
 #if CRT_COOP_STATS
   fprintf(stderr, "[coop stats] closest: %llu walks, %llu iterations, %llu box tests, %llu triangle tests | shadow: %llu walks, %llu iterations, %llu box tests, %llu triangle tests\n",
-          st[32], st[34], st[35], st[36], st[33], st[37], st[38], st[39]);
+          st[CRT_STAT_HANDOFF_CLOSEST], st[CRT_STAT_COOP_DEBUG], st[CRT_STAT_COOP_DEBUG + 1], st[CRT_STAT_COOP_DEBUG + 2],
+          st[CRT_STAT_HANDOFF_SHADOW], st[CRT_STAT_COOP_DEBUG + 3], st[CRT_STAT_COOP_DEBUG + 4], st[CRT_STAT_COOP_DEBUG + 5]);
 #endif
   if (timed) {
     float ms = 0.f;
@@ -1936,6 +1911,42 @@ static int collect_stats_one(crtb200_ctx *c, bool timed) {
   return CRTB200_OK;
 }
 
+// the counters of one render (not its times) added into running totals
+static void add_counts(crtb200_stats &t, SideCounts &tx, const crtb200_stats &s, const SideCounts &sx) {
+  t.rays_primary += s.rays_primary;
+  t.rays_shadow += s.rays_shadow;
+  t.rays_reflection += s.rays_reflection;
+  t.rays_refraction += s.rays_refraction;
+  t.node_tests_closest += s.node_tests_closest;
+  t.triangle_tests_closest += s.triangle_tests_closest;
+  t.node_tests_shadow += s.node_tests_shadow;
+  t.triangle_tests_shadow += s.triangle_tests_shadow;
+  t.handoff_closest += s.handoff_closest;
+  t.handoff_shadow += s.handoff_shadow;
+  t.shadow_rays_zero_term += s.shadow_rays_zero_term;
+  t.kernel_launches += s.kernel_launches;
+  tx.diffuse += sx.diffuse;
+  tx.px_samples += sx.px_samples;
+  tx.stopped += sx.stopped;
+}
+
+// counters of the primary plus those of the peers (rays, tests, launches); times are the primary's (fork to join)
+static int collect_stats(crtb200_ctx *c) {
+  int rc = collect_stats_one(c, true);
+  if (rc) return rc;
+  for (crtb200_ctx *p : c->peers) {
+    if (!p->last_pending) continue;
+    CUDA_TRY(cudaSetDevice(p->device));
+    CUDA_TRY(cudaStreamSynchronize(p->stream));
+    rc = collect_stats_one(p, false);
+    p->last_pending = false;
+    if (rc) return rc;
+    add_counts(c->last, c->last_side, p->last, p->last_side);
+  }
+  CUDA_TRY(cudaSetDevice(c->device));
+  return CRTB200_OK;
+}
+
 extern "C" {
 
 int crtb200_render(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_options *o, float *rgb_out,
@@ -1951,19 +1962,17 @@ int crtb200_render(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_opti
   c->last = crtb200_stats{};
   // Rectangle grids that leave pixels uncovered keep the previous frame there (colorBuffer persistence), so the whole
   // persistent frame is copied after the render; otherwise each chunk's band is copied as soon as it is stored.
-  const bool shard = o->shard_count > 1;
-  HostOut host;
-  host.rgb = rgb_out;
-  host.rgb8 = rgb8_out;
-  host.hits = hits_out;
+  const HostOut host{rgb_out, rgb8_out, hits_out};
   int rc = plan_mask(c, o);
   if (rc) return rc;
-  const bool want_bands = !shard && !c->mask_needed && (rgb_out || rgb8_out || hits_out);
-  bool banded = false;
-  rc = enqueue_any(c, cam, o, c->frame.p, rgb8_out ? c->frame8.p : nullptr, hits_out ? c->hits.p : nullptr, nullptr,
-                   c->stream, true, want_bands ? &host : nullptr, &banded);
+  FrameReq r(cam, o);
+  r.d_rgb = c->frame.p;
+  r.d_rgb8 = rgb8_out ? c->frame8.p : nullptr;
+  r.d_hits = hits_out ? c->hits.p : nullptr;
+  if (o->shard_count <= 1 && !c->mask_needed && (rgb_out || rgb8_out || hits_out)) r.host = &host;
+  rc = enqueue_any(c, r, c->stream);
   if (rc) return rc;
-  if (!banded) {
+  if (!c->bands_copied) {
     if (rgb_out) CUDA_TRY(cudaMemcpyAsync(rgb_out, c->frame.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
     if (rgb8_out) CUDA_TRY(cudaMemcpyAsync(rgb8_out, c->frame8.p, px * 3, cudaMemcpyDeviceToHost, c->stream));
     if (hits_out) CUDA_TRY(cudaMemcpyAsync(hits_out, c->hits.p, px * sizeof(HitRec), cudaMemcpyDeviceToHost, c->stream));
@@ -1971,10 +1980,10 @@ int crtb200_render(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_opti
   const double enqueue_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
   CUDA_TRY(cudaStreamSynchronize(c->stream));
   const double sync_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-  rc = collect_stats(c, true);
+  rc = collect_stats(c);
   if (rc) return rc;
   c->last.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-  if (banded && c->dbg_chunks && getenv("CRT_CHUNK_TIMES")) {
+  if (c->bands_copied && c->dbg_chunks && getenv("CRT_CHUNK_TIMES")) {
     fprintf(stderr, "[chunk times] host: enqueue %.3f ms, synchronised %.3f ms, stats read %.3f ms; device frame %.3f ms\n", enqueue_ms, sync_ms,
             c->last.total_ms, c->last.device_ms);
     for (uint32_t k = 0; k < c->dbg_chunks; k++) {
@@ -1989,24 +1998,13 @@ int crtb200_render(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_opti
   return CRTB200_OK;
 }
 
-static void add_stats(crtb200_stats &total, const crtb200_stats &s) {
-  total.rays_primary += s.rays_primary;
-  total.rays_shadow += s.rays_shadow;
-  total.rays_reflection += s.rays_reflection;
-  total.rays_refraction += s.rays_refraction;
-  total.node_tests_closest += s.node_tests_closest;
-  total.triangle_tests_closest += s.triangle_tests_closest;
-  total.node_tests_shadow += s.node_tests_shadow;
-  total.triangle_tests_shadow += s.triangle_tests_shadow;
-  total.handoff_closest += s.handoff_closest;
-  total.handoff_shadow += s.handoff_shadow;
-  total.shadow_rays_zero_term += s.shadow_rays_zero_term;
+static void add_stats(crtb200_stats &total, SideCounts &tx, const crtb200_stats &s, const SideCounts &sx) {
+  add_counts(total, tx, s, sx);
   total.device_ms += s.device_ms;
   total.closest_ms += s.closest_ms;
   total.shadow_ms += s.shadow_ms;
   total.coop_closest_ms += s.coop_closest_ms;
   total.coop_shadow_ms += s.coop_shadow_ms;
-  total.kernel_launches += s.kernel_launches;
   total.levels = s.levels;
 }
 
@@ -2032,18 +2030,17 @@ int crtb200_render_frames(crtb200_ctx *c, const crtb200_camera *cams, uint32_t n
   if (rc) return rc;
   if (c->mask_needed || o->shard_count > 1 || o->count_work != 0 || n_frames < 2) {
     crtb200_stats total{};
-    uint64_t diffuse = 0;
+    SideCounts side;
     for (uint32_t f = 0; f < n_frames; f++) {
       crtb200_stats s{};
       set_frame_offset(c, f);
       rc = crtb200_render(c, cams + f, o, rgb_out ? rgb_out + f * px * 3 : nullptr, rgb8_out ? rgb8_out + f * px * 3 : nullptr, nullptr, &s);
       set_frame_offset(c, 0);
       if (rc) return rc;
-      add_stats(total, s);
-      diffuse += c->last_diffuse;
+      add_stats(total, side, s, c->last_side);
     }
     total.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    c->last_diffuse = diffuse;
+    c->last_side = side;
     if (stats) *stats = total;
     return CRTB200_OK;
   }
@@ -2062,7 +2059,11 @@ int crtb200_render_frames(crtb200_ctx *c, const crtb200_camera *cams, uint32_t n
     uint8_t *d_rgb8 = rgb8_out ? (k ? c->frame8_b.p : c->frame8.p) : nullptr;
     if (f >= 2) CUDA_TRY(cudaStreamWaitEvent(c->stream, c->copied[k], 0));  // this pair's previous frame has left the device
     set_frame_offset(c, f);
-    rc = enqueue_any(c, cams + f, o, d_rgb, d_rgb8, nullptr, nullptr, c->stream, true, nullptr, nullptr, f > 0);
+    FrameReq r(cams + f, o);
+    r.d_rgb = d_rgb;
+    r.d_rgb8 = d_rgb8;
+    r.batch_continuation = f > 0;
+    rc = enqueue_any(c, r, c->stream);
     set_frame_offset(c, 0);
     if (rc) return rc;
     launches += c->last.kernel_launches;
@@ -2078,7 +2079,7 @@ int crtb200_render_frames(crtb200_ctx *c, const crtb200_camera *cams, uint32_t n
     std::swap(c->frame, c->frame_b);
     std::swap(c->frame8, c->frame8_b);
   }
-  rc = collect_stats(c, true);
+  rc = collect_stats(c);
   if (rc) return rc;
   c->last.kernel_launches = launches;
   c->last.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -2094,14 +2095,16 @@ int crtb200_render_device(crtb200_ctx *c, const crtb200_camera *cam, const crtb2
   const uint32_t shard_count = o->shard_count ? o->shard_count : 1;
   c->last = crtb200_stats{};
   c->last_pending = true;
-  if (shard_count > 1 && o->shard_full_frame)  // the shard's pixels at their place in a full frame (peer-mapped, crtb200_ipc_open)
-    return enqueue_frame(c, cam, o, d_rgb_out, d_rgb8_out, nullptr, nullptr, (cudaStream_t)stream, true);
-  if (shard_count > 1) {
+  FrameReq r(cam, o);
+  if (shard_count > 1 && !o->shard_full_frame) {
     // sharded: d_rgb_out is the shard's compact slab (crtb200_shard_items x 3 floats), see crtb200_assemble_shards
     if (d_rgb8_out) return fail(CRTB200_ERR_ARG, "sharded rendering writes a float slab only");
-    return enqueue_frame(c, cam, o, nullptr, nullptr, nullptr, d_rgb_out, (cudaStream_t)stream, true);
+    r.d_slab = d_rgb_out;
+  } else {  // (shard_full_frame: the shard's pixels at their place in a full frame, peer-mapped, crtb200_ipc_open)
+    r.d_rgb = d_rgb_out;
+    r.d_rgb8 = d_rgb8_out;
   }
-  return enqueue_any(c, cam, o, d_rgb_out, d_rgb8_out, nullptr, nullptr, (cudaStream_t)stream, true);
+  return enqueue_any(c, r, (cudaStream_t)stream);  // (a tile shard goes to enqueue_frame)
 }
 
 // ---- progressive sessions (DESIGN.md 3.10.1) ---------------------------------------------------------------------
@@ -2110,19 +2113,15 @@ int crtb200_render_device(crtb200_ctx *c, const crtb200_camera *cam, const crtb2
 // context's sampling stay as they are.  As in enqueue_any, the peers start after c->stream has reached this point and
 // c->stream continues after every peer's kernel.
 static int shard_pass(crtb200_ctx *c, const std::function<void(crtb200_ctx *, const Frame &, cudaStream_t)> &launch) {
-  const uint32_t n = 1u + (uint32_t)c->peers.size();
+  const std::vector<crtb200_ctx *> gpus = all_gpus(c);
+  const uint32_t n = (uint32_t)gpus.size();
   if (n > 1) CUDA_TRY(cudaEventRecord(c->multi_fork, c->stream));
   for (uint32_t i = 0; i < n; i++) {
-    crtb200_ctx *x = i ? c->peers[i - 1] : c;
+    crtb200_ctx *x = gpus[i];
     CUDA_TRY(cudaSetDevice(x->device));
     const int rc = plan_mask(x, &c->acc_opt);
     if (rc) return rc;
-    Frame fr{};
-    fr.tiles_x = (x->sc.width + 7) / 8;
-    fr.n_tiles = fr.tiles_x * ((x->sc.height + 3) / 4);
-    fr.shard_index = i;
-    fr.shard_count = n;
-    fr.mask = x->mask_needed ? x->mask.p : nullptr;
+    Frame fr = frame_tiles(x, i, n);
     fr.n_items0 = shard_item_count(x, i, n);
     if (i) CUDA_TRY(cudaStreamWaitEvent(x->stream, c->multi_fork, 0));
     launch(x, fr, x->stream);
@@ -2203,9 +2202,10 @@ static int accum_begin(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_
   c->acc_smp = *s;
   c->acc_smp.use_gi = 1;
   c->acc_smp.rays_per_pixel = 1;  // unused: a step says how many samples it renders
-  const uint32_t n = 1u + (uint32_t)c->peers.size();
+  const std::vector<crtb200_ctx *> gpus = all_gpus(c);
+  const uint32_t n = (uint32_t)gpus.size();
   for (uint32_t i = 0; i < n; i++) {
-    crtb200_ctx *x = i ? c->peers[i - 1] : c;
+    crtb200_ctx *x = gpus[i];
     const size_t items = std::max<size_t>(1, shard_item_count(c, i, n));
     cudaError_t e = cudaSetDevice(x->device);
     if (e == cudaSuccess) e = x->acc_sum.ensure(items);
@@ -2261,22 +2261,21 @@ int crtb200_accum_step(crtb200_ctx *c, uint32_t n_samples, crtb200_stats *stats)
   const AccumPass a{c->acc_done, n_samples, c->acc_adaptive ? &c->acc_ap : nullptr};
   // The session's sampling stands in for the context's during the step, because queue planning and the Philox key both
   // read ctx->sampling; frame_offset is 0 outside crtb200_render_frames, so the key is the session's frame_index.
+  const std::vector<crtb200_ctx *> gpus = all_gpus(c);
   std::vector<crtb200_sampling> saved;
-  for (size_t i = 0; i <= c->peers.size(); i++) {
-    crtb200_ctx *x = i ? c->peers[i - 1] : c;
-    saved.push_back(x->sampling);
-    x->sampling = c->acc_smp;
-  }
-  int rc = enqueue_any(c, &c->acc_cam, &c->acc_opt, nullptr, nullptr, nullptr, nullptr, c->stream, true, nullptr, nullptr, false, &a);
-  for (size_t i = 0; i <= c->peers.size(); i++) (i ? c->peers[i - 1] : c)->sampling = saved[i];
+  for (crtb200_ctx *x : gpus) saved.push_back(std::exchange(x->sampling, c->acc_smp));
+  FrameReq r(&c->acc_cam, &c->acc_opt);
+  r.acc = &a;
+  int rc = enqueue_any(c, r, c->stream);
+  for (size_t i = 0; i < gpus.size(); i++) gpus[i]->sampling = saved[i];
   if (rc) return rc;
   CUDA_TRY(cudaStreamSynchronize(c->stream));
-  rc = collect_stats(c, true);
+  rc = collect_stats(c);
   if (rc) return rc;
   c->acc_done += n_samples;
   if (c->acc_adaptive) {
-    c->acc_px_samples += c->last_px_samples;
-    c->acc_active_px -= c->last_stopped;
+    c->acc_px_samples += c->last_side.px_samples;
+    c->acc_active_px -= c->last_side.stopped;
   }
   c->last.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
   if (stats) *stats = c->last;
@@ -2420,7 +2419,7 @@ int crtb200_last_stats(crtb200_ctx *c, crtb200_stats *stats) {
   CUDA_TRY(cudaSetDevice(c->device));
   if (c->last_pending) {
     CUDA_TRY(cudaEventSynchronize(c->ev[1]));
-    int rc = collect_stats(c, true);
+    int rc = collect_stats(c);
     if (rc) return rc;
     c->last_pending = false;
   }
@@ -2480,12 +2479,10 @@ int crtb200_assemble_shards(crtb200_ctx *c, const float *d_slabs, uint32_t shard
   CUDA_TRY(cudaSetDevice(c->device));
   uint32_t items = 0;
   crtb200_shard_items(c, shard_count, &items);
-  Frame fr{};
-  fr.tiles_x = (c->sc.width + 7) / 8;
-  fr.n_tiles = fr.tiles_x * ((c->sc.height + 3) / 4);
   // rectangle lists that leave pixels uncovered: the assembled frame keeps what d_rgb_out held there (colorBuffer
-  // persistence), exactly like the unsharded path -- the mask is the one of the last render's rectangle list
-  fr.mask = c->mask_needed ? c->mask.p : nullptr;
+  // persistence), exactly like the unsharded path -- the mask is the one of the last render's rectangle list.
+  // k_assemble sets the shard of each item itself.
+  const Frame fr = frame_tiles(c, 0, shard_count);
   k_assemble<<<c->sm_count * 8, 256, 0, (cudaStream_t)stream>>>(c->sc, fr, d_slabs, items, shard_count, d_rgb_out, d_rgb8_out);
   CUDA_TRY(cudaGetLastError());
   return CRTB200_OK;
