@@ -4,7 +4,8 @@
 //   K2  k_closest                   persistent closest-hit traversal, one ray per lane, stack-free two-level KD walk
 //   K4/K5 k_shade                   per-hit: barycentrics, smooth normal, texture sample, material switch,
 //                                   reflect / refract + Fresnel, compaction of children into the next level's queue
-//   K3  k_shadow                    persistent any-hit traversal, one (diffuse hit, light) pair per lane -> visibility
+//   K3  k_shadow                    persistent any-hit traversal, one (diffuse hit, light) pair per lane -> visibility;
+//                                   K2 and K3 run one loop (walk_loop) with a walk kind each
 //   K2b/K3b k_coop                  the walks K2 / K3 hand off once their queue is dry: one warp per walk, a LIFO of
 //                                   subtrees in shared memory; an early pass runs next to the traversal kernel
 //                                   (k_mark tells it that the kernel has ended), a final pass behind both
@@ -124,6 +125,14 @@ CRT_DI uint32_t warp_alloc(uint32_t *counter, uint32_t n) {
   if (lane_id() == 31 && total) base = atomicAdd(counter, total);
   base = __shfl_sync(CRT_FULL_MASK, base, 31);
   return base + incl - n;
+}
+
+// Adds a per-lane counter, summed over the (fully converged) warp, to stats[slot]: one atomic per warp, none for a zero sum.
+template <class T>
+CRT_DI void warp_stat_add(const Levels &lv, const uint32_t slot, T v) {
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(CRT_FULL_MASK, v, d);
+  if (lane_id() == 0 && v) atomicAdd(&lv.stats[slot], (unsigned long long)v);
 }
 
 // level-0 work item -> pixel.  Items are numbered tile-major (8x4 tiles) so a warp starts on one coherent tile.
@@ -377,8 +386,7 @@ CRT_DI bool tail_handoff(const Levels &lv, const uint32_t launch, const bool wan
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// K2: closest hit.  Replaces RayTracer::trace -> KDTree<ObjectKDTreeSubTree>::intersect -> KDTree<Triangle>::intersect
-// (RayTracer.cpp:453-458, KDTree.cpp:127-166, 48-87).
+// The persistent traversal loop of K2 (k_closest) and K3 (k_shadow).
 //
 // Persistent warps, one ray per lane.  Every loop below has a WARP-UNIFORM trip count (its condition is a vote), so the
 // 32 lanes stay converged under independent thread scheduling; per-lane work is predicated.  (A first version with
@@ -390,33 +398,34 @@ CRT_DI bool tail_handoff(const Levels &lv, const uint32_t launch, const bool wan
 //   tri phase     tri_phase: the parked ranges, packed across the warp
 // MODE: 2 = this loop.  (0 = while-while and 1 = merged single loop were the round-1 predecessors; their measurements are
 // in profiles/r1_tuning.md, their code is gone.)
-// ------------------------------------------------------------------------------------------------------------
-// JITTER (PRIMARY only): level 0 of a GI frame, jittered primary rays (a template flag, so that the unsampled primary
-// kernels keep their register allocation)
-template <bool PRIMARY, bool COUNT, int REFILL, int MODE, bool CULL, bool WIDE, bool JITTER = false>
-__global__ void __launch_bounds__(CRT_TRAV_BLOCK, PRIMARY ? CRT_TRAV_MIN_BLOCKS : CRT_TRAV_MIN_BLOCKS_SEC) k_closest(const DScene sc, const Frame fr, const Levels lv, const uint32_t level,
-                                                uint32_t *__restrict__ work_counter) {
-  static_assert(MODE == 2, "only loop mode 2 is implemented");
-  __shared__ WarpShare s_ws[CRT_TRAV_BLOCK / 32];
-  WarpShare *ws = &s_ws[threadIdx.x >> 5];
-  const uint32_t total = PRIMARY ? level0_items<JITTER>(fr) : lv.counts[level];
-  const uint32_t node_base = lv.offset[level];
+//
+// A walk kind (ClosestWalk, ShadowWalk) holds the per-lane state of a walk's answer and supplies the steps that differ.
+// `id` is where the answer goes (the ray's queue node / the pair's visibility slot), also the hand-off record's id:
+//   total, take(i, ray, id)  work items of the launch; the ray of item i (false: the item is answered without a walk)
+//   begin(ray, i, id)        a new walk's answer state; tri_dist() = w of its entry in the warp's ray table
+//   limit(), allow_behind()  the node phase's culling bound (node_test)
+//   tri()                    the triangle phase; true when the lane's answer can no longer change
+//   answer(), handoff()      the result of a finished walk; the record of a walk handed to k_coop (tail_handoff)
+//   finish(lv)               the walk kind's own counters
+//   SHADOW                   also the index of its CRT_PHASE_CLOCKS records; STAT_NODES / STAT_TRIS: its COUNT slots
+// SKIPR, DEDUP: trav_slow's; COUNT: count node and triangle tests; HANDOFF: hand long walks to k_coop once the queue is
+// dry; EARLY: end a walk as soon as tri() reports its answer final.
+template <int REFILL, bool CULL, bool WIDE, bool SKIPR, int DEDUP, bool COUNT, bool HANDOFF, bool EARLY, class W>
+CRT_DI void walk_loop(const DScene &sc, const Frame &fr, const Levels &lv, uint32_t *work_counter, WarpShare &ws, W &w) {
+  const uint32_t total = w.total;
   const uint32_t lane = lane_id();
-  const uint32_t tail_start = COUNT ? CRT_INVALID : tail_policy(lv, total, false);
+  const uint32_t tail_start = HANDOFF ? tail_policy(lv, total, W::SHADOW) : CRT_INVALID;
   const uint32_t poll_mask = tail_poll_mask(total);
   bool active = false, exhausted = false, closed = false;
-  uint32_t node = 0, n_nodes = 0, n_tris = 0, round = 0, walk_iters = 0, dry_rounds = 0;
+  uint32_t id = 0, n_nodes = 0, n_tris = 0, round = 0, walk_iters = 0, dry_rounds = 0;
 #if CRT_PHASE_CLOCKS
   uint32_t ray_iters = 0;
 #endif
   Ray ray;
   Trav tv;
-  Closest cl;
-  tv.tref = tv.tend = 0;
   ray.o = ray.d = ray.inv = mk(0.f, 0.f, 0.f);
   ray.flags = 0;
   trav_begin<WIDE>(tv, sc);
-  closest_begin(cl);
   CRT_PC_DECL
   for (;;) {
     CRT_PC_MARK(4)
@@ -432,105 +441,145 @@ __global__ void __launch_bounds__(CRT_TRAV_BLOCK, PRIMARY ? CRT_TRAV_MIN_BLOCKS 
         exhausted = true;
       }
       const uint32_t i = start + __popc(idle & lanemask_lt());
-      if (!active && i < total) {
-        bool valid = true;
-        if (PRIMARY) {
-          uint32_t row, col;
-          valid = item_pixel<JITTER>(fr, sc, fr.item_begin + i, row, col);
-          if (valid) {
-            if (JITTER)
-              jittered_primary_ray(fr, sc.width, sc.height, row, col, ray.o, ray.d);
-            else
-              primary_ray(fr.cam, sc.width, sc.height, row, col, ray.o, ray.d);
-          }
-        } else {
-          const float4 o = lv.ray_o[node_base - lv.offset[1] + i];
-          const float4 d = lv.ray_d[node_base - lv.offset[1] + i];
-          ray.o = mk(o.x, o.y, o.z);
-          ray.d = mk(d.x, d.y, d.z);
-        }
-        if (valid) {
-          ray_prepare(ray, PRIMARY);
-          trav_begin<WIDE>(tv, sc);
-          closest_begin(cl);
-          node = node_base + i;
-          active = true;
-          walk_iters = 0;
+      if (!active && i < total && w.take(sc, fr, lv, i, ray, id)) {
+        ray_prepare(ray, W::PRIMARY);
+        trav_begin<WIDE>(tv, sc);
+        w.begin(ray, i, id);
+        active = true;
+        walk_iters = 0;
 #if CRT_PHASE_CLOCKS
-          ray_iters = 0;
+        ray_iters = 0;
 #endif
-          if (MODE == 2) {
-            ws->ro[lane] = make_float4(ray.o.x, ray.o.y, ray.o.z, 0.f);
-            ws->rd[lane] = make_float4(ray.d.x, ray.d.y, ray.d.z, 0.f);
-          }
-        }
+        ws.ro[lane] = make_float4(ray.o.x, ray.o.y, ray.o.z, w.tri_dist());
+        ws.rd[lane] = make_float4(ray.d.x, ray.d.y, ray.d.z, 0.f);
       }
     }
-    if (!COUNT && tail_start != CRT_INVALID) {
+    if (HANDOFF && tail_start != CRT_INVALID) {
       if (!exhausted && (++round & poll_mask) == 0u) exhausted = queue_dry(work_counter);
       if (exhausted && !closed) {
         const uint32_t thr = tail_threshold(lv, tail_start, dry_rounds++);
-        if (tail_handoff(lv, level, active && walk_iters >= thr, node, tv, cl.best_t, cl.best_tri, closed)) active = false;
+        if (w.handoff(lv, active && walk_iters >= thr, id, tv, closed)) active = false;
       }
     }
     if (!__any_sync(CRT_FULL_MASK, active)) {
       if (exhausted) break;
       continue;
     }
-    if (MODE == 2) {
-      CRT_PC_MARK(0)
-      CRT_PC_TAIL(exhausted, active)
-      // ---- between-trees bookkeeping for lanes whose cursor ran off a tree (rare) ----
-      for (;;) {
-        const bool slow = active && tv.tref == tv.tend && tv.cur == tv.cend;
-        if (!__any_sync(CRT_FULL_MASK, slow)) break;
-        if (slow && trav_slow<false, (COUNT ? 0 : (WIDE ? 2 : 1)), CULL>(tv, sc, ray) == TRAV_DONE) {
-          lv.hit_tri[node] = cl.best_tri;
-          lv.hit_t[node] = cl.best_t;
-          active = false;
-          CRT_PC_RAY_DONE(0, ray_iters)
-        }
+    CRT_PC_MARK(0)
+    CRT_PC_TAIL(exhausted, active)
+    // ---- between-trees bookkeeping for lanes whose cursor ran off a tree (rare) ----
+    for (;;) {
+      const bool slow = active && tv.tref == tv.tend && tv.cur == tv.cend;
+      if (!__any_sync(CRT_FULL_MASK, slow)) break;
+      if (slow && trav_slow<SKIPR, DEDUP, CULL>(tv, sc, ray) == TRAV_DONE) {
+        w.answer(lv, id);
+        active = false;
+        CRT_PC_RAY_DONE(W::SHADOW, ray_iters)
       }
-      CRT_PC_MARK(1)
-      // ---- node phase: one AABB step per iteration while enough lanes want one ----
-      bool need = active && tv.tref == tv.tend;
-      const uint32_t thr = node_threshold(__popc(__ballot_sync(CRT_FULL_MASK, active)));
-      while ((uint32_t)__popc(__ballot_sync(CRT_FULL_MASK, need)) >= thr) {
-        CRT_PC_COUNT(5, 1)
+    }
+    CRT_PC_MARK(1)
+    // ---- node phase: one AABB step per iteration while enough lanes want one ----
+    bool need = active && tv.tref == tv.tend;
+    const uint32_t thr = node_threshold(__popc(__ballot_sync(CRT_FULL_MASK, active)));
+    while ((uint32_t)__popc(__ballot_sync(CRT_FULL_MASK, need)) >= thr) {
+      CRT_PC_COUNT(5, 1)
 #if CRT_PHASE_CLOCKS
-        if (need) ray_iters++;
+      if (need) ray_iters++;
 #endif
-        if (need) {
-          walk_iters++;
-          // conservative culling: beyond the best finite hit; behind the origin once a finite hit exists (crt_device.cuh)
-          const bool fin = cl.min_t < CRT_INF;
-          need = CRT_NODE_PAIR ? trav_fast2<COUNT, CULL>(tv, sc, ray, n_nodes, cl.min_t, fin) : trav_fast<COUNT, CULL>(tv, sc, ray, n_nodes, cl.min_t, fin);
-        }
+      if (need) {
+        walk_iters++;
+        need = CRT_NODE_PAIR ? trav_fast2<COUNT, CULL>(tv, sc, ray, n_nodes, w.limit(), w.allow_behind())
+                             : trav_fast<COUNT, CULL>(tv, sc, ray, n_nodes, w.limit(), w.allow_behind());
       }
-      CRT_PC_MARK(2)
-      // ---- triangle phase: all pending leaves, packed across the warp ----
-      const bool parked = active && tv.tref != tv.tend;
-      if (__any_sync(CRT_FULL_MASK, parked)) {
-        bool dummy = false;
-        CRT_PC_COUNT(6, 1)
-        tri_phase<false, PRIMARY, COUNT>(sc, *ws, parked, !__any_sync(CRT_FULL_MASK, need), tv.tref, tv.tend, cl, dummy, n_tris);
-      }
-      CRT_PC_MARK(3)
     }
+    CRT_PC_MARK(2)
+    // ---- triangle phase: all pending leaves, packed across the warp ----
+    const bool parked = active && tv.tref != tv.tend;
+    if (__any_sync(CRT_FULL_MASK, parked)) {
+      CRT_PC_COUNT(6, 1)
+      const bool done = w.template tri<COUNT>(sc, ws, parked, !__any_sync(CRT_FULL_MASK, need), tv, n_tris);
+      if (EARLY && active && done) {  // early termination: the rest of the walk cannot change the answer
+        tv.tref = tv.tend = 0;
+        w.answer(lv, id);
+        active = false;
+        CRT_PC_RAY_DONE(W::SHADOW, ray_iters)
+      }
+    }
+    CRT_PC_MARK(3)
   }
-  CRT_PC_FLUSH(CRT_STAT_PHASE)
+  CRT_PC_FLUSH(CRT_STAT_PHASE + 8 * W::SHADOW)
+  w.finish(lv);
   if (COUNT) {
-    unsigned long long a = n_nodes, b = n_tris;
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) {
-      a += __shfl_xor_sync(CRT_FULL_MASK, a, d);
-      b += __shfl_xor_sync(CRT_FULL_MASK, b, d);
-    }
-    if (lane == 0) {
-      atomicAdd(&lv.stats[CRT_STAT_NODES_CLOSEST], a);
-      atomicAdd(&lv.stats[CRT_STAT_TRIS_CLOSEST], b);
-    }
+    warp_stat_add(lv, W::STAT_NODES, (unsigned long long)n_nodes);
+    warp_stat_add(lv, W::STAT_TRIS, (unsigned long long)n_tris);
   }
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// K2: closest hit.  Replaces RayTracer::trace -> KDTree<ObjectKDTreeSubTree>::intersect -> KDTree<Triangle>::intersect
+// (RayTracer.cpp:453-458, KDTree.cpp:127-166, 48-87).  Work item = one ray of `level` (level 0: a pixel of the chunk);
+// the answer is the ray node's hit_tri / hit_t.
+// JITTER (PRIMARY only): level 0 of a GI frame, jittered primary rays (a template flag, so that the unsampled primary
+// kernels keep their register allocation)
+// ------------------------------------------------------------------------------------------------------------
+template <bool P, bool JITTER>
+struct ClosestWalk {
+  static constexpr bool PRIMARY = P, SHADOW = false;
+  static constexpr uint32_t STAT_NODES = CRT_STAT_NODES_CLOSEST, STAT_TRIS = CRT_STAT_TRIS_CLOSEST;
+  const uint32_t level, total, node_base;
+  Closest cl;
+  CRT_DI ClosestWalk(const Frame &fr, const Levels &lv, const uint32_t lvl)
+      : level(lvl), total(PRIMARY ? level0_items<JITTER>(fr) : lv.counts[lvl]), node_base(lv.offset[lvl]) {
+    closest_begin(cl);
+  }
+  CRT_DI bool take(const DScene &sc, const Frame &fr, const Levels &lv, const uint32_t i, Ray &ray, uint32_t &) const {
+    if (!PRIMARY) {
+      const float4 o = lv.ray_o[node_base - lv.offset[1] + i];
+      const float4 d = lv.ray_d[node_base - lv.offset[1] + i];
+      ray.o = mk(o.x, o.y, o.z);
+      ray.d = mk(d.x, d.y, d.z);
+      return true;
+    }
+    uint32_t row, col;
+    if (!item_pixel<JITTER>(fr, sc, fr.item_begin + i, row, col)) return false;
+    if (JITTER)
+      jittered_primary_ray(fr, sc.width, sc.height, row, col, ray.o, ray.d);
+    else
+      primary_ray(fr.cam, sc.width, sc.height, row, col, ray.o, ray.d);
+    return true;
+  }
+  CRT_DI void begin(const Ray &, const uint32_t i, uint32_t &node) {
+    closest_begin(cl);
+    node = node_base + i;
+  }
+  CRT_DI float tri_dist() const { return 0.f; }
+  // conservative culling: beyond the best finite hit; behind the origin once a finite hit exists (crt_device.cuh)
+  CRT_DI float limit() const { return cl.min_t; }
+  CRT_DI bool allow_behind() const { return cl.min_t < CRT_INF; }
+  template <bool COUNT>
+  CRT_DI bool tri(const DScene &sc, WarpShare &ws, const bool parked, const bool flush, Trav &tv, uint32_t &n_tris) {
+    bool dummy = false;
+    tri_phase<false, PRIMARY, COUNT>(sc, ws, parked, flush, tv.tref, tv.tend, cl, dummy, n_tris);
+    return false;
+  }
+  CRT_DI void answer(const Levels &lv, const uint32_t node) const {
+    lv.hit_tri[node] = cl.best_tri;
+    lv.hit_t[node] = cl.best_t;
+  }
+  CRT_DI bool handoff(const Levels &lv, const bool want, const uint32_t node, const Trav &tv, bool &closed) const {
+    return tail_handoff(lv, level, want, node, tv, cl.best_t, cl.best_tri, closed);
+  }
+  CRT_DI void finish(const Levels &) const {}
+};
+
+template <bool PRIMARY, bool COUNT, int REFILL, int MODE, bool CULL, bool WIDE, bool JITTER = false>
+__global__ void __launch_bounds__(CRT_TRAV_BLOCK, PRIMARY ? CRT_TRAV_MIN_BLOCKS : CRT_TRAV_MIN_BLOCKS_SEC) k_closest(const DScene sc, const Frame fr, const Levels lv, const uint32_t level,
+                                                uint32_t *__restrict__ work_counter) {
+  static_assert(MODE == 2, "only loop mode 2 is implemented");
+  __shared__ WarpShare s_ws[CRT_TRAV_BLOCK / 32];
+  WarpShare &ws = s_ws[threadIdx.x >> 5];
+  ClosestWalk<PRIMARY, JITTER> w(fr, lv, level);
+  walk_loop<REFILL, CULL, WIDE, false, (COUNT ? 0 : (WIDE ? 2 : 1)), COUNT, !COUNT, false>(sc, fr, lv, work_counter, ws, w);
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -758,24 +807,10 @@ __global__ void __launch_bounds__(256) k_shade(const DScene sc, const Frame fr, 
     }
   }
   // ray statistics (traced rays only, SURVEY 8(d))
-  unsigned long long a = n_prim, b = n_refl, c = n_refr;
-#pragma unroll
-  for (int s = 16; s > 0; s >>= 1) {
-    a += __shfl_xor_sync(CRT_FULL_MASK, a, s);
-    b += __shfl_xor_sync(CRT_FULL_MASK, b, s);
-    c += __shfl_xor_sync(CRT_FULL_MASK, c, s);
-  }
-  if (lane_id() == 0) {
-    if (a) atomicAdd(&lv.stats[CRT_STAT_RAYS_PRIMARY], a);
-    if (b) atomicAdd(&lv.stats[CRT_STAT_RAYS_REFLECTION], b);
-    if (c) atomicAdd(&lv.stats[CRT_STAT_RAYS_REFRACTION], c);
-  }
-  if (GI) {
-    unsigned long long g = n_diff;
-#pragma unroll
-    for (int s = 16; s > 0; s >>= 1) g += __shfl_xor_sync(CRT_FULL_MASK, g, s);
-    if (lane_id() == 0 && g) atomicAdd(&lv.stats[CRT_STAT_DIFFUSE], g);
-  }
+  warp_stat_add(lv, CRT_STAT_RAYS_PRIMARY, (unsigned long long)n_prim);
+  warp_stat_add(lv, CRT_STAT_RAYS_REFLECTION, (unsigned long long)n_refl);
+  warp_stat_add(lv, CRT_STAT_RAYS_REFRACTION, (unsigned long long)n_refr);
+  if (GI) warp_stat_add(lv, CRT_STAT_DIFFUSE, (unsigned long long)n_diff);
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -787,7 +822,7 @@ __global__ void __launch_bounds__(256) k_shade(const DScene sc, const Frame fr, 
 // light from neighbouring hits; the result is one visibility byte per pair.  (One item per pair, not per hit: the
 // kernel's tail is its longest item, profiles/r1_tuning.md.)
 // COUNT: 0 = no counters; 1 = count under the reference's visit-all rule (early termination disabled, same result);
-// 2 = count the work this kernel really does with early termination.  Loop structure: see k_closest.
+// 2 = count the work this kernel really does with early termination.
 // ------------------------------------------------------------------------------------------------------------
 CRT_DI void shadow_ray_setup(const DScene &sc, const Frame &fr, const V3 P, const V3 N, const uint32_t light, Ray &ray,
                              float &dist, float &contrib) {
@@ -809,6 +844,59 @@ CRT_DI float shadow_limit(const Ray &ray, const float dist) {
   return dist * 1.0001f + 1e-4f + 1e-6f * (fabsf(ray.o.x) + fabsf(ray.o.y) + fabsf(ray.o.z));
 }
 
+// ZERO_TERMS: a pair whose light term is exactly zero may be answered without a walk (not in the visit-all counting mode)
+template <bool ZERO_TERMS>
+struct ShadowWalk {
+  static constexpr bool PRIMARY = false, SHADOW = true;
+  static constexpr uint32_t STAT_NODES = CRT_STAT_NODES_SHADOW, STAT_TRIS = CRT_STAT_TRIS_SHADOW;
+  const uint32_t n_hits, total;
+  uint32_t n_moot = 0;
+  float dist = 0.0f, t_limit = 0.0f;
+  bool occluded = false;
+  CRT_DI ShadowWalk(const DScene &sc, const Levels &lv) : n_hits(lv.counts[CRT_MAX_LEVELS]), total(n_hits * sc.n_lights) {}
+  CRT_DI bool take(const DScene &sc, const Frame &fr, const Levels &lv, const uint32_t i, Ray &ray, uint32_t &slot) {
+    const uint32_t light = i / n_hits, hit = i - light * n_hits;
+    const float4 q0 = lv.dq[3 * (size_t)hit], q1 = lv.dq[3 * (size_t)hit + 1];
+    float contrib;
+    shadow_ray_setup(sc, fr, mk(q0.x, q0.y, q0.z), mk(q1.x, q1.y, q1.z), light, ray, dist, contrib);
+    slot = hit * sc.n_lights + light;
+    // A light term that is exactly zero needs no walk.  The reference traces the shadow ray of every (hit, light) pair
+    // (RayTracer.cpp:314-317) and then adds `direct * albedo` with direct = float(I) / area * max(0, L.N)
+    // (:313, :320-327): for a surface turned away from the light direct is +0, the term is (+-0, +-0, +-0) for any
+    // finite albedo / texel, and x + (+-0) == x bit for bit (the sum starts at +0): visible or not, the pixel is the
+    // same.  The pair still counts as a traced ray (ray counts are the reference's).
+    bool moot = false;
+    if (ZERO_TERMS && lv.skip_zero_terms && contrib == 0.0f) {
+      const float4 q2 = lv.dq[3 * (size_t)hit + 2];
+      const uint32_t nf = 0x7f800000u;
+      moot = (__float_as_uint(q1.w) & nf) != nf && (__float_as_uint(q2.x) & nf) != nf && (__float_as_uint(q2.y) & nf) != nf;
+    }
+    if (moot) {
+      lv.vis[slot] = 0;
+      n_moot++;
+    }
+    return !moot;
+  }
+  CRT_DI void begin(const Ray &ray, const uint32_t, uint32_t &) {
+    t_limit = shadow_limit(ray, dist);
+    occluded = false;
+  }
+  CRT_DI float tri_dist() const { return dist; }
+  CRT_DI float limit() const { return t_limit; }
+  CRT_DI bool allow_behind() const { return true; }
+  template <bool COUNT>
+  CRT_DI bool tri(const DScene &sc, WarpShare &ws, const bool parked, const bool flush, Trav &tv, uint32_t &n_tris) {
+    Closest unused;
+    tri_phase<true, false, COUNT>(sc, ws, parked, flush, tv.tref, tv.tend, unused, occluded, n_tris);
+    return occluded;
+  }
+  CRT_DI void answer(const Levels &lv, const uint32_t slot) const { lv.vis[slot] = occluded ? 0 : 1; }
+  CRT_DI bool handoff(const Levels &lv, const bool want, const uint32_t slot, const Trav &tv, bool &closed) const {
+    return tail_handoff(lv, CRT_MAX_LEVELS, want, slot, tv, 0.0f, CRT_INVALID, closed);
+  }
+  CRT_DI void finish(const Levels &lv) const { warp_stat_add(lv, CRT_STAT_ZERO_TERM, n_moot); }
+};
+
 // SKIPR: shadow rays ignore refractive meshes, as the reference does only when !useGI (AccelerationStructure.cpp:67-71);
 // GI frames instantiate SKIPR = false.
 template <int COUNT, int REFILL, int MODE, bool CULL, bool WIDE, bool SKIPR = true>
@@ -816,147 +904,10 @@ __global__ void __launch_bounds__(CRT_TRAV_BLOCK, CRT_TRAV_MIN_BLOCKS) k_shadow(
                                                                              uint32_t *__restrict__ work_counter) {
   static_assert(MODE == 2, "only loop mode 2 is implemented");
   __shared__ WarpShare s_ws[CRT_TRAV_BLOCK / 32];
-  WarpShare *ws = &s_ws[threadIdx.x >> 5];
-  const uint32_t n_hits = lv.counts[CRT_MAX_LEVELS];
-  const uint32_t total = n_hits * sc.n_lights;
-  const uint32_t lane = lane_id();
-  const uint32_t tail_start = COUNT ? CRT_INVALID : tail_policy(lv, total, true);
-  const uint32_t poll_mask = tail_poll_mask(total);
-  bool active = false, exhausted = false, occluded = false, closed = false;
-  uint32_t slot = 0, n_nodes = 0, n_tris = 0, round = 0, walk_iters = 0, dry_rounds = 0, n_moot = 0;
-#if CRT_PHASE_CLOCKS
-  uint32_t ray_iters = 0;
-#endif
-  float dist = 0.0f, t_limit = 0.0f;
-  Ray ray;
-  Trav tv;
-  ray.o = ray.d = ray.inv = mk(0.f, 0.f, 0.f);
-  ray.flags = 0;
-  trav_begin<WIDE>(tv, sc);
-  CRT_PC_DECL
-  for (;;) {
-    CRT_PC_MARK(4)
-    CRT_PC_COUNT(7, 1)
-    const uint32_t idle = __ballot_sync(CRT_FULL_MASK, !active);
-    if (!exhausted && __popc(idle) >= REFILL) {
-      const uint32_t want = __popc(idle);
-      uint32_t start = 0;
-      if (lane == 0) start = atomicAdd(work_counter, want);
-      start = __shfl_sync(CRT_FULL_MASK, start, 0);
-      if (start + want >= total) {
-        if (!exhausted && start < total) queue_mark_dry(work_counter);  // (the warp that takes the last rays)
-        exhausted = true;
-      }
-      const uint32_t i = start + __popc(idle & lanemask_lt());
-      if (!active && i < total) {
-        const uint32_t light = i / n_hits, hit = i - light * n_hits;
-        const float4 q0 = lv.dq[3 * (size_t)hit], q1 = lv.dq[3 * (size_t)hit + 1];
-        float contrib;
-        shadow_ray_setup(sc, fr, mk(q0.x, q0.y, q0.z), mk(q1.x, q1.y, q1.z), light, ray, dist, contrib);
-        slot = hit * sc.n_lights + light;
-        // A light term that is exactly zero needs no walk.  The reference traces the shadow ray of every (hit, light) pair
-        // (RayTracer.cpp:314-317) and then adds `direct * albedo` with direct = float(I) / area * max(0, L.N)
-        // (:313, :320-327): for a surface turned away from the light direct is +0, the term is (+-0, +-0, +-0) for any
-        // finite albedo / texel, and x + (+-0) == x bit for bit (the sum starts at +0): visible or not, the pixel is the
-        // same.  The pair still counts as a traced ray (ray counts are the reference's).  Not in the visit-all counting
-        // mode, which reproduces the reference's work.
-        bool moot = false;
-        if (COUNT != 1 && lv.skip_zero_terms && contrib == 0.0f) {
-          const float4 q2 = lv.dq[3 * (size_t)hit + 2];
-          const uint32_t nf = 0x7f800000u;
-          moot = (__float_as_uint(q1.w) & nf) != nf && (__float_as_uint(q2.x) & nf) != nf && (__float_as_uint(q2.y) & nf) != nf;
-        }
-        if (moot) {
-          lv.vis[slot] = 0;
-          n_moot++;
-        } else {
-          ray_prepare(ray, false);
-          trav_begin<WIDE>(tv, sc);
-          t_limit = shadow_limit(ray, dist);
-          occluded = false;
-          active = true;
-          walk_iters = 0;
-#if CRT_PHASE_CLOCKS
-          ray_iters = 0;
-#endif
-          if (MODE == 2) {
-            ws->ro[lane] = make_float4(ray.o.x, ray.o.y, ray.o.z, dist);
-            ws->rd[lane] = make_float4(ray.d.x, ray.d.y, ray.d.z, 0.f);
-          }
-        }
-      }
-    }
-    if (COUNT == 0 && tail_start != CRT_INVALID) {
-      if (!exhausted && (++round & poll_mask) == 0u) exhausted = queue_dry(work_counter);
-      if (exhausted && !closed) {
-        const uint32_t thr = tail_threshold(lv, tail_start, dry_rounds++);
-        if (tail_handoff(lv, CRT_MAX_LEVELS, active && walk_iters >= thr, slot, tv, 0.0f, CRT_INVALID, closed)) active = false;
-      }
-    }
-    if (!__any_sync(CRT_FULL_MASK, active)) {
-      if (exhausted) break;
-      continue;
-    }
-    if (MODE == 2) {
-      CRT_PC_MARK(0)
-      CRT_PC_TAIL(exhausted, active)
-      for (;;) {
-        const bool slow = active && tv.tref == tv.tend && tv.cur == tv.cend;
-        if (!__any_sync(CRT_FULL_MASK, slow)) break;
-        if (slow && trav_slow<SKIPR, (COUNT == 1 ? 0 : (WIDE ? 2 : 1)), CULL>(tv, sc, ray) == TRAV_DONE) {
-          lv.vis[slot] = occluded ? 0 : 1;
-          active = false;
-          CRT_PC_RAY_DONE(1, ray_iters)
-        }
-      }
-      CRT_PC_MARK(1)
-      bool need = active && tv.tref == tv.tend;
-      const uint32_t thr = node_threshold(__popc(__ballot_sync(CRT_FULL_MASK, active)));
-      while ((uint32_t)__popc(__ballot_sync(CRT_FULL_MASK, need)) >= thr) {
-        CRT_PC_COUNT(5, 1)
-#if CRT_PHASE_CLOCKS
-        if (need) ray_iters++;
-#endif
-        if (need) {
-          walk_iters++;
-          need = CRT_NODE_PAIR ? trav_fast2<(COUNT != 0), CULL>(tv, sc, ray, n_nodes, t_limit, true) : trav_fast<(COUNT != 0), CULL>(tv, sc, ray, n_nodes, t_limit, true);
-        }
-      }
-      CRT_PC_MARK(2)
-      const bool parked = active && tv.tref != tv.tend;
-      if (__any_sync(CRT_FULL_MASK, parked)) {
-        CRT_PC_COUNT(6, 1)
-        Closest unused;
-        tri_phase<true, false, (COUNT != 0)>(sc, *ws, parked, !__any_sync(CRT_FULL_MASK, need), tv.tref, tv.tend, unused, occluded, n_tris);
-        if (COUNT != 1 && active && occluded) {  // early termination: the rest of the walk cannot change the answer
-          tv.tref = tv.tend = 0;
-          lv.vis[slot] = 0;
-          active = false;
-          CRT_PC_RAY_DONE(1, ray_iters)
-        }
-      }
-      CRT_PC_MARK(3)
-    }
-  }
-  CRT_PC_FLUSH(CRT_STAT_PHASE + 8)
-  {
-    uint32_t m = n_moot;
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) m += __shfl_xor_sync(CRT_FULL_MASK, m, d);
-    if (lane == 0 && m) atomicAdd(&lv.stats[CRT_STAT_ZERO_TERM], (unsigned long long)m);
-  }
-  if (COUNT) {
-    unsigned long long a = n_nodes, b = n_tris;
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) {
-      a += __shfl_xor_sync(CRT_FULL_MASK, a, d);
-      b += __shfl_xor_sync(CRT_FULL_MASK, b, d);
-    }
-    if (lane == 0) {
-      atomicAdd(&lv.stats[CRT_STAT_NODES_SHADOW], a);
-      atomicAdd(&lv.stats[CRT_STAT_TRIS_SHADOW], b);
-    }
-  }
+  WarpShare &ws = s_ws[threadIdx.x >> 5];
+  ShadowWalk<COUNT != 1> w(sc, lv);
+  walk_loop<REFILL, CULL, WIDE, SKIPR, (COUNT == 1 ? 0 : (WIDE ? 2 : 1)), (COUNT != 0), COUNT == 0, COUNT != 1>(
+      sc, fr, lv, work_counter, ws, w);
 }
 
 // ------------------------------------------------------------------------------------------------------------
