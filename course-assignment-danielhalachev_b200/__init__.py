@@ -12,7 +12,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-from typing import Optional, Sequence
+from typing import NamedTuple, Optional, Sequence
 
 import numpy as np
 
@@ -145,6 +145,21 @@ class Stats(C.Structure):
         return d
 
 
+class RayBatch(C.Structure):
+    """crtb200_ray_batch: a batch of caller-supplied rays in device memory (crtb200_trace_rays_device)."""
+    _fields_ = [("n", C.c_uint32), ("ray_type", C.c_uint32), ("traversal", C.c_uint32), ("count_work", C.c_uint32),
+                ("rays", C.c_void_p), ("max_distance", C.c_void_p), ("hits", C.c_void_p), ("occluded", C.c_void_p)]
+
+
+class Hits(NamedTuple):
+    """Closest hits of Context.trace: mesh, triangle and t are views of `records`, one (..., 3) int32 tensor in the
+    crtb200_hit layout; t holds float32 bits (t.view(torch.float32))."""
+    mesh: "object"
+    triangle: "object"
+    t: "object"
+    records: "object"
+
+
 class Sampling(C.Structure):
     """crtb200_sampling: GI + jittered supersampling under the project's sampling contract (DESIGN.md 3.10)."""
     _fields_ = [("use_gi", C.c_uint32), ("gi_samples", C.c_uint32), ("rays_per_pixel", C.c_uint32),
@@ -222,6 +237,9 @@ def core() -> C.CDLL:
         lib.crtb200_ipc_close.argtypes = [C.c_int, C.c_void_p]
         lib.crtb200_generate_rays.argtypes = [C.c_void_p, C.POINTER(Camera), C.c_void_p]
         lib.crtb200_trace_rays.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.crtb200_trace_rays_device.argtypes = [C.c_void_p, C.POINTER(RayBatch), C.c_void_p]
+        lib.crtb200_generate_rays_device.argtypes = [C.c_void_p, C.POINTER(Camera), C.c_void_p, C.c_void_p]
+        lib.crtb200_last_query_stats.argtypes = [C.c_void_p, C.POINTER(Stats)]
         lib.crtb200_device_count.argtypes = [C.POINTER(C.c_int)]
         lib.crtb200_debug_powf5.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]
         lib.crtb200_upload_geometry.argtypes = [C.c_void_p, C.POINTER(Scene)]
@@ -612,6 +630,88 @@ class Context:
         hits = np.zeros(n, HIT_DTYPE)
         _check_core(core().crtb200_trace_rays(self._h, rays.ctypes.data, n, ray_type, traversal, None, hits.ctypes.data, None))
         return hits
+
+    def _first_device(self):
+        import torch
+        return torch.device("cuda", self.devices()[0])
+
+    def generate_rays_device(self, camera: Camera):
+        """Camera rays of every pixel as an (H, W, 6) float32 CUDA tensor on the context's first device (origin xyz,
+        direction xyz; the layout of generate_rays), written on torch.cuda.current_stream() without a host round trip."""
+        import torch
+        dev = self._first_device()
+        out = torch.empty((self.height, self.width, 6), dtype=torch.float32, device=dev)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _check_core(core().crtb200_generate_rays_device(self._h, C.byref(camera), out.data_ptr() or None, stream or None))
+        return out
+
+    def trace(self, rays, ray_type: int, max_distance=None, traversal: int = 0, count_work: int = 0, out=None):
+        """Traces a batch of caller-supplied rays on the GPU (crtb200_trace_rays_device), on torch.cuda.current_stream().
+
+        rays: float32 CUDA tensor of shape (..., 6) on the context's first device, contiguous in its last dimension
+        (origin xyz, direction xyz; directions of any length).  ray_type RAY_PRIMARY / RAY_REFLECTION / RAY_REFRACTION
+        returns the closest hits as Hits(mesh, triangle, t, records): views of records, one (..., 3) int32 tensor (t: float32 bits,
+        hits.t.view(torch.float32); a miss is -1, -1, 0); RAY_SHADOW needs max_distance (float32, the leading shape) and
+        returns a uint8 tensor of the leading shape, 1 where some candidate lies within max_distance.  out= reuses a
+        previous result's storage: the (..., 3) int32 tensor (or a Hits of it), or the uint8 tensor.  Asynchronous like
+        any CUDA work on the stream; query_stats() synchronises."""
+        import torch
+        dev = self._first_device()
+
+        def need(t, what, dtype, shape):
+            if not isinstance(t, torch.Tensor):
+                raise CrtError(f"{what} must be a torch tensor")
+            if t.dtype != dtype:
+                raise CrtError(f"{what} must be {dtype}, not {t.dtype}")
+            if t.device != dev:
+                raise CrtError(f"{what} must be on {dev}, not {t.device}")
+            if tuple(t.shape) != tuple(shape):
+                raise CrtError(f"{what} must have shape {tuple(shape)}, not {tuple(t.shape)}")
+
+        if not isinstance(rays, torch.Tensor) or rays.dim() < 1 or rays.shape[-1] != 6:
+            raise CrtError("rays must be a torch tensor of shape (..., 6)")
+        lead = tuple(rays.shape[:-1])
+        need(rays, "rays", torch.float32, lead + (6,))
+        if ray_type not in (RAY_PRIMARY, RAY_SHADOW, RAY_REFLECTION, RAY_REFRACTION):
+            raise CrtError(f"ray_type {ray_type} has no query (primary, shadow, reflection or refraction)")
+        if rays.numel() and rays.stride(-1) != 1:
+            raise CrtError("rays must be contiguous in its last dimension")
+        n = rays.numel() // 6
+        if n >= 1 << 31:
+            raise CrtError(f"a ray batch holds fewer than 2^31 rays, not {n}")
+        flat = rays.reshape(-1, 6).contiguous()  # (a copy on the stream only when the leading dimensions are strided)
+        b = RayBatch(n=n, ray_type=ray_type, traversal=traversal, count_work=count_work, rays=flat.data_ptr() or None)
+        if ray_type == RAY_SHADOW:
+            if max_distance is None:
+                raise CrtError("a shadow query needs max_distance")
+            need(max_distance, "max_distance", torch.float32, lead)
+            md = max_distance.contiguous()
+            res = out if out is not None else torch.empty(lead, dtype=torch.uint8, device=dev)
+            need(res, "out", torch.uint8, lead)
+            if not res.is_contiguous():
+                raise CrtError("out must be contiguous")
+            b.max_distance, b.occluded = md.data_ptr() or None, res.data_ptr() or None
+        else:
+            buf = out.records if isinstance(out, Hits) else out
+            res = buf if buf is not None else torch.empty(lead + (3,), dtype=torch.int32, device=dev)
+            need(res, "out", torch.int32, lead + (3,))
+            if not res.is_contiguous():
+                raise CrtError("out must be contiguous")
+            b.hits = res.data_ptr() or None
+        if n:
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            _check_core(core().crtb200_trace_rays_device(self._h, C.byref(b), stream or None))
+        if ray_type == RAY_SHADOW:
+            return res
+        return Hits(res[..., 0], res[..., 1], res[..., 2], res)
+
+    def query_stats(self) -> dict:
+        """Statistics of the last trace() / trace_rays() (crtb200_last_query_stats; waits for the query to finish): rays
+        of its type, node / triangle tests under its count_work, handoff_closest / handoff_shadow, device_ms,
+        kernel_launches."""
+        st = Stats()
+        _check_core(core().crtb200_last_query_stats(self._h, C.byref(st)))
+        return st.as_dict()
 
     def debug_powf5(self, x: np.ndarray) -> np.ndarray:
         x = np.ascontiguousarray(x, dtype=np.float32)

@@ -388,7 +388,8 @@ CRT_DI bool node_test(const float4 lo, const float4 hi, const Ray &r, const floa
   return pass;
 }
 
-// One traversal micro-step.  Returns 0 = keep stepping, 1 = a triangle list is pending (tref..tend), 2 = traversal
+// One traversal micro-step of the walk (trav_fast / trav_fast2 for an AABB step, trav_slow between trees): the state
+// transitions of KDTree.cpp:48-87 / 127-166.  trav_slow returns TRAV_STEP = keep stepping or TRAV_DONE = traversal
 // complete.  Top-level and mesh-level AABB tests share one code path so lanes at different levels do not diverge.
 //   SKIP_REFRACTIVE  shadow rays ignore refractive meshes (AccelerationStructure.cpp:67-71).
 //   DEDUP            a mesh listed in several top-level leaves is traversed once per ray instead of once per listing.
@@ -401,41 +402,12 @@ enum { TRAV_STEP = 0, TRAV_LEAF = 1, TRAV_DONE = 2 };
 template <bool SKIP_REFRACTIVE, int DEDUP, bool CULL>
 CRT_DI int trav_slow(Trav &s, const DScene &sc, const Ray &r);
 
-template <bool SKIP_REFRACTIVE, bool COUNT, int DEDUP, bool CULL>
-CRT_DI int trav_step(Trav &s, const DScene &sc, const Ray &r, uint32_t &node_tests, const float limit, const bool allow_behind) {
-  if (s.cur != s.cend) {
-    const uint32_t idx = s.cur;
-    const float4 lo = ld_node(&sc.nodes[2 * (size_t)idx]);
-    const float4 hi = ld_node(&sc.nodes[2 * (size_t)idx + 1]);
-    const uint32_t a = __float_as_uint(lo.w);
-    const bool leaf = (a & CRT_LEAF_FLAG) != 0u;
-    if (COUNT) node_tests++;
-    const bool pass = node_test<CULL>(lo, hi, r, s.mu, limit, allow_behind);
-    s.cur = (pass || leaf) ? idx + 1 : a;
-    if (pass && leaf) {
-      const uint32_t first = __float_as_uint(hi.w), last = first + (a & ~CRT_LEAF_FLAG);
-      if (s.below) {
-        s.tref = first;
-        s.tend = last;
-        return TRAV_LEAF;
-      }
-      s.mref = first;  // a top-level leaf: remember where to continue, then walk its meshes
-      s.mend = last;
-      s.resume = s.cur;
-      s.cur = s.cend;
-      s.below = 1u;
-    }
-    return TRAV_STEP;
-  }
-  return trav_slow<SKIP_REFRACTIVE, DEDUP, CULL>(s, sc, r);
-}
-
-// trav_step split in two for the MODE 2 kernels (crt_kernels.cuh), whose tight node loop only wants the AABB step:
+// The step split in two for the MODE 2 kernels (crt_kernels.cuh), whose tight node loop only wants the AABB step:
 //   trav_fast   one AABB test for a lane with cur != cend.  Returns true while the lane can take another fast step;
 //               false when a triangle range is pending (tref..tend) or the cursor ran off its tree (trav_slow is due).
 //   trav_slow   the bookkeeping between trees for a lane with cur == cend and no pending triangles: next mesh of the
 //               current top-level leaf, or back to the top-level tree, or TRAV_DONE.
-// Together they perform exactly the state transitions of trav_step.
+// Together they perform exactly the state transitions of the reference's walk.
 template <bool COUNT, bool CULL>
 CRT_DI bool trav_fast(Trav &s, const DScene &sc, const Ray &r, uint32_t &node_tests, const float limit, const bool allow_behind) {
   const uint32_t idx = s.cur;
@@ -511,8 +483,8 @@ CRT_DI bool trav_fast2(Trav &s, const DScene &sc, const Ray &r, uint32_t &node_t
 }
 
 // DEDUP: 0 = every listing of a mesh is walked (the reference's work; counting mode), 1 = visited-mesh set in the 64-bit
-// register Trav::seen (scenes with <= 64 meshes), 2 = in shared memory (65..512 meshes; kernels instantiated WIDE),
-// 3 = whichever of the two the scene asks for (k_query: not a hot kernel).  Scenes with more meshes than that walk
+// register Trav::seen (scenes with <= 64 meshes), 2 = in shared memory (65..512 meshes; kernels instantiated WIDE).
+// Scenes with more meshes than that walk
 // every listing -- correct (the candidates repeat and a repeat never wins a strict <), only slower.
 template <bool SKIP_REFRACTIVE, int DEDUP, bool CULL>
 CRT_DI int trav_slow(Trav &s, const DScene &sc, const Ray &r) {

@@ -12,6 +12,9 @@
 //   K3c k_accumulate                in-order light sum per diffuse hit
 //   K6  k_resolve                   bottom-up combine of the ray tree in the reference's expression order
 //   K7  k_store                     level-0 colours -> framebuffer (f32 + PPMColor u8)
+//   Q   k_query_closest / k_query_shadow / k_coop_query
+//                                   caller-supplied ray batches on the same loop and hand-off (walk kinds
+//                                   QueryClosestWalk / QueryShadowWalk, k_coop's body with the ray source CoopQuerySrc)
 //
 // Reference functions replaced are cited at each kernel.  No tensor cores: the path is pointer-chasing + scalar
 // binary32 arithmetic; the B200-specific choices are the 32-byte-sector node records, L2-resident working set,
@@ -1017,14 +1020,48 @@ __global__ void k_mark(uint32_t *flag) {
   if (threadIdx.x == 0) *reinterpret_cast<volatile uint32_t *>(flag) = 1u;
 }
 
-// SKIPR: shadow rays ignore refractive meshes (false in GI frames, see k_shadow)
-template <bool SHADOW, bool PRIMARY, bool CULL, int GW, bool SKIPR = true>
-__global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_coop(const DScene sc, const Frame fr, const Levels lv, const uint32_t level, const uint32_t early) {
+// Where k_coop's walks come from and where their answers go (the ray source of coop_walks):
+//   ray<SHADOW, PRIMARY>(sc, lv, id, ray, dist)  the ray of record id (and, SHADOW, its distance bound)
+//   shadow_limit(ray, dist)                      the culling bound of a shadow walk (CULL)
+//   shadow_answer(lv, id, occluded)              closest_answer(sc, lv, id, cl)
+// CoopFrameSrc: the walks of a frame's traversal launches (queue nodes / visibility slots); CoopQuerySrc (below, with
+// the query kernels): a caller's ray batch.
+struct CoopFrameSrc {
+  const Frame &fr;
+  template <bool SHADOW, bool PRIMARY>
+  CRT_DI void ray(const DScene &sc, const Levels &lv, const uint32_t id, Ray &ray, float &dist) const {
+    if (SHADOW) {
+      const uint32_t hit = id / sc.n_lights, light = id - hit * sc.n_lights;
+      const float4 q0 = lv.dq[3 * (size_t)hit], q1 = lv.dq[3 * (size_t)hit + 1];
+      float contrib;
+      shadow_ray_setup(sc, fr, mk(q0.x, q0.y, q0.z), mk(q1.x, q1.y, q1.z), light, ray, dist, contrib);
+    } else if (PRIMARY) {
+      uint32_t row, col;
+      item_pixel<true>(fr, sc, fr.item_begin + (id - lv.offset[0]), row, col);  // valid: the main kernel started this ray
+      if (fr.gi)
+        jittered_primary_ray(fr, sc.width, sc.height, row, col, ray.o, ray.d);
+      else
+        primary_ray(fr.cam, sc.width, sc.height, row, col, ray.o, ray.d);
+    } else {
+      const float4 o = lv.ray_o[id - lv.offset[1]], d = lv.ray_d[id - lv.offset[1]];
+      ray.o = mk(o.x, o.y, o.z);
+      ray.d = mk(d.x, d.y, d.z);
+    }
+  }
+  CRT_DI float shadow_limit(const Ray &ray, const float dist) const { return crtd::shadow_limit(ray, dist); }
+  CRT_DI void shadow_answer(const Levels &lv, const uint32_t id, const bool occluded) const { lv.vis[id] = occluded ? 0 : 1; }
+  CRT_DI void closest_answer(const DScene &, const Levels &lv, const uint32_t id, const Closest &cl) const {
+    lv.hit_tri[id] = cl.best_tri;
+    lv.hit_t[id] = cl.best_t;
+  }
+};
+
+// The body of k_coop and k_coop_query.  SKIPR: shadow rays ignore refractive meshes (false in GI frames, see k_shadow)
+template <bool SHADOW, bool PRIMARY, bool CULL, int GW, bool SKIPR, class Src>
+CRT_DI void coop_walks(const DScene &sc, const Levels &lv, const uint32_t level, const uint32_t early, WarpCoop &wc, const Src &src) {
   constexpr uint32_t NG = 32u / GW;            // walks per warp
   constexpr uint32_t CAP = CRT_COOP_CAP / NG;  // LIFO entries per walk
   static_assert(GW == 8 || GW == 16 || GW == 32, "group width");
-  __shared__ WarpCoop s_wc[CRT_COOP_WARPS];
-  WarpCoop &wc = s_wc[threadIdx.x >> 5];
   const uint32_t lane = lane_id(), gl = lane & (GW - 1u), g0 = lane & ~(GW - 1u);
   const uint32_t gm = (GW == 32 ? CRT_FULL_MASK : ((1u << GW) - 1u)) << g0;  // lanes of this group
   uint32_t *const stack = wc.stack + (g0 / GW) * CAP;
@@ -1082,23 +1119,7 @@ __global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_co
       } else if (got != CRT_INVALID) {
         const uint4 r0 = __ldcg(&lv.ovf[3 * (size_t)r]), r1 = __ldcg(&lv.ovf[3 * (size_t)r + 1]), r2 = __ldcg(&lv.ovf[3 * (size_t)r + 2]);
         id = got;
-        if (SHADOW) {
-          const uint32_t hit = id / sc.n_lights, light = id - hit * sc.n_lights;
-          const float4 q0 = lv.dq[3 * (size_t)hit], q1 = lv.dq[3 * (size_t)hit + 1];
-          float contrib;
-          shadow_ray_setup(sc, fr, mk(q0.x, q0.y, q0.z), mk(q1.x, q1.y, q1.z), light, ray, dist, contrib);
-        } else if (PRIMARY) {
-          uint32_t row, col;
-          item_pixel<true>(fr, sc, fr.item_begin + (id - lv.offset[0]), row, col);  // valid: the main kernel started this ray
-          if (fr.gi)
-            jittered_primary_ray(fr, sc.width, sc.height, row, col, ray.o, ray.d);
-          else
-            primary_ray(fr.cam, sc.width, sc.height, row, col, ray.o, ray.d);
-        } else {
-          const float4 o = lv.ray_o[id - lv.offset[1]], d = lv.ray_d[id - lv.offset[1]];
-          ray.o = mk(o.x, o.y, o.z);
-          ray.d = mk(d.x, d.y, d.z);
-        }
+        src.template ray<SHADOW, PRIMARY>(sc, lv, id, ray, dist);
         ray_prepare(ray, PRIMARY);
         // the walk's state where the main kernel left it
         cur = r0.y;
@@ -1112,7 +1133,7 @@ __global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_co
         cl.best_t = __uint_as_float(r2.z);
         cl.best_tri = r2.w;
         cl.min_t = (cl.best_tri != CRT_INVALID && cl.best_t < CRT_INF) ? cl.best_t : CRT_INF;
-        lim = SHADOW ? shadow_limit(ray, dist) : cl.min_t;
+        lim = SHADOW ? src.shadow_limit(ray, dist) : cl.min_t;
         occluded = false;
         in_mesh = false;
         busy = true;
@@ -1120,7 +1141,7 @@ __global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_co
     }
     if (!__any_sync(CRT_FULL_MASK, busy)) break;  // idle groups have just found the record list empty
 
-    // ---- 2. between mesh walks: one step of the ray's itinerary (trav_step's order of events, per group) ----
+    // ---- 2. between mesh walks: one step of the ray's itinerary (trav_fast / trav_slow's order of events, per group) ----
     if (busy && !in_mesh) {
       if (cur < cend) {
         if (below) {
@@ -1181,12 +1202,10 @@ __global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_co
       } else {
         // itinerary complete
         if (gl == 0) {
-          if (SHADOW) {
-            lv.vis[id] = 1;
-          } else {
-            lv.hit_tri[id] = cl.best_tri;
-            lv.hit_t[id] = cl.best_t;
-          }
+          if (SHADOW)
+            src.shadow_answer(lv, id, false);
+          else
+            src.closest_answer(sc, lv, id, cl);
         }
         busy = false;
       }
@@ -1298,7 +1317,7 @@ __global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_co
         }
       }
       if (SHADOW && occluded) {  // the first occluder ends the record (SURVEY App. A-11)
-        if (gl == 0) lv.vis[id] = 0;
+        if (gl == 0) src.shadow_answer(lv, id, true);
         busy = false;
         in_mesh = false;
         __syncwarp(gm);
@@ -1316,6 +1335,12 @@ __global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_co
   atomicAdd(&lv.stats[CRT_STAT_COOP_DEBUG + (SHADOW ? 4 : 1)], dbg_nodes);
   atomicAdd(&lv.stats[CRT_STAT_COOP_DEBUG + (SHADOW ? 5 : 2)], dbg_tris);
 #endif
+}
+
+template <bool SHADOW, bool PRIMARY, bool CULL, int GW, bool SKIPR = true>
+__global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_coop(const DScene sc, const Frame fr, const Levels lv, const uint32_t level, const uint32_t early) {
+  __shared__ WarpCoop s_wc[CRT_COOP_WARPS];
+  coop_walks<SHADOW, PRIMARY, CULL, GW, SKIPR>(sc, lv, level, early, s_wc[threadIdx.x >> 5], CoopFrameSrc{fr});
 }
 
 // K3c: the light loop of RayTracer::calculateDiffusion (RayTracer.cpp:308-330): per diffuse hit, walk the lights IN
@@ -1787,7 +1812,7 @@ __global__ void __launch_bounds__(256) k_powf5(const float *__restrict__ x, uint
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) out[i] = crt_powf5(x[i]);
 }
 
-// K1 standalone: RayTracer::getRay + shootRay's re-normalisation, for the ray parity test.
+// K1 standalone: RayTracer::getRay + shootRay's re-normalisation into a caller's array (crtb200_generate_rays_device).
 __global__ void __launch_bounds__(256) k_generate_rays(const DScene sc, const DCamera cam, float *__restrict__ rays) {
   const uint32_t n = sc.width * sc.height;
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
@@ -1803,58 +1828,162 @@ __global__ void __launch_bounds__(256) k_generate_rays(const DScene sc, const DC
   }
 }
 
-// Caller-supplied rays: RayTracer::trace / RayTracer::hasIntersection as plain queries (one ray per thread).
-__global__ void __launch_bounds__(256) k_query(const DScene sc, const float *__restrict__ rays, uint32_t n,
-                                              uint32_t ray_type, const float *__restrict__ max_distance,
-                                              HitRec *__restrict__ hits, uint8_t *__restrict__ occluded) {
-  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    Ray ray;
-    ray.o = mk(rays[6 * (size_t)i], rays[6 * (size_t)i + 1], rays[6 * (size_t)i + 2]);
-    ray.d = mk(rays[6 * (size_t)i + 3], rays[6 * (size_t)i + 4], rays[6 * (size_t)i + 5]);
-    ray_prepare(ray, ray_type == 0u);
-    Trav tv;
-    trav_begin<true>(tv, sc);
-    uint32_t dummy = 0;
-    if (ray_type == 1u) {
-      const float dist = max_distance[i];
-      bool occ = false;
-      for (;;) {
-        int st = TRAV_STEP;
-        while (st == TRAV_STEP) st = trav_step<true, false, 3, false>(tv, sc, ray, dummy, 0.0f, false);
-        if (st == TRAV_DONE || occ) break;
-        while (tv.tref != tv.tend) {
-          const uint32_t tri = __ldg(&sc.leaf_refs[tv.tref++]);
-          float t;
-          V3 p;
-          if (triangle_test(__ldg(&sc.tri_geom[3 * (size_t)tri]), __ldg(&sc.tri_geom[3 * (size_t)tri + 1]),
-                            __ldg(&sc.tri_geom[3 * (size_t)tri + 2]), ray, t, p)) {
-            if (vlen(vsub(p, ray.o)) <= dist) occ = true;
-          }
-        }
-      }
-      occluded[i] = occ ? 1 : 0;
-    } else {
-      Closest cl;
-      closest_begin(cl);
-      for (;;) {
-        int st = TRAV_STEP;
-        while (st == TRAV_STEP) st = trav_step<false, false, 3, false>(tv, sc, ray, dummy, 0.0f, false);
-        if (st == TRAV_DONE) break;
-        while (tv.tref != tv.tend) {
-          const uint32_t tri = __ldg(&sc.leaf_refs[tv.tref++]);
-          float t;
-          V3 p;
-          if (triangle_test(__ldg(&sc.tri_geom[3 * (size_t)tri]), __ldg(&sc.tri_geom[3 * (size_t)tri + 1]),
-                            __ldg(&sc.tri_geom[3 * (size_t)tri + 2]), ray, t, p))
-            closest_offer(cl, tri, t);
-        }
-      }
-      HitRec h;
-      public_tri(sc, cl.best_tri, h);
-      h.t = cl.best_tri == CRT_INVALID ? 0.0f : cl.best_t;
-      hits[i] = h;
-    }
+// ------------------------------------------------------------------------------------------------------------
+// Caller-supplied ray batches (crtb200_trace_rays_device, DESIGN.md 3.12): RayTracer::trace (RayTracer.cpp:453-458) and
+// the non-GI RayTracer::hasIntersection (RayTracer.cpp:507-518) for rays the caller holds in device memory, walked by
+// the same persistent loop as K2 / K3 (walk kinds QueryClosestWalk / QueryShadowWalk) and handed off to the same k_coop
+// body (ray source CoopQuerySrc).  Work item i = ray i of the batch; its answer goes straight to the caller's arrays.
+// ------------------------------------------------------------------------------------------------------------
+struct QueryBatch {
+  const float *rays;          // n x 6: origin xyz, direction xyz
+  const float *max_distance;  // n, shadow queries
+  HitRec *hits;               // n, closest-hit queries (public numbering; miss: -1, -1, t = 0)
+  uint8_t *occluded;          // n, shadow queries
+  uint32_t n;
+};
+
+// Ray i of a batch: three 8-byte loads when the array is 8-byte aligned (a ray is 24 bytes)
+CRT_DI void query_ray(const float *rays, const uint32_t i, Ray &ray) {
+  const float *r = rays + 6 * (size_t)i;
+  if ((reinterpret_cast<uintptr_t>(rays) & 7u) == 0u) {
+    const float2 a = *reinterpret_cast<const float2 *>(r), b = *reinterpret_cast<const float2 *>(r + 2),
+                 c = *reinterpret_cast<const float2 *>(r + 4);
+    ray.o = mk(a.x, a.y, b.x);
+    ray.d = mk(b.y, c.x, c.y);
+  } else {
+    ray.o = mk(r[0], r[1], r[2]);
+    ray.d = mk(r[3], r[4], r[5]);
   }
+}
+
+// The culling bound of a caller's shadow ray.  shadow_limit assumes |d| = 1 within 2 ulp; a caller's direction may
+// have any length, so the *beyond* skip is applied only when the computed |d| is within 8 ulp of 1 (then the true |d| is
+// within 11 ulp of 1, far inside shadow_limit's 1e-4 relative slack); other rays keep *behind* alone (DESIGN.md 3.12).
+CRT_DI float query_shadow_limit(const Ray &ray, const float dist) {
+  return fabsf(fsub(vlen(ray.d), 1.0f)) <= 8.0f * CRT_FLT_EPSILON ? shadow_limit(ray, dist) : CRT_INF;
+}
+
+CRT_DI void query_store_hit(const DScene &sc, HitRec *hits, const uint32_t i, const uint32_t tri, const float t) {
+  HitRec h;
+  public_tri(sc, tri, h);
+  h.t = tri == CRT_INVALID ? 0.0f : t;
+  hits[i] = h;
+}
+
+// Closest hit of ray i; PRIMARY (CRTB200_RAY_PRIMARY): the primary ray's back-face rule (Ray.cpp:13).  Limits as
+// ClosestWalk's: culling in parameter space holds for any direction length (DESIGN.md 3.12).
+template <bool P>
+struct QueryClosestWalk {
+  static constexpr bool PRIMARY = P, SHADOW = false;
+  static constexpr uint32_t STAT_NODES = CRT_STAT_NODES_CLOSEST, STAT_TRIS = CRT_STAT_TRIS_CLOSEST;
+  const DScene &sc;
+  const QueryBatch &qb;
+  const uint32_t total;
+  Closest cl;
+  CRT_DI QueryClosestWalk(const DScene &s, const QueryBatch &b) : sc(s), qb(b), total(b.n) { closest_begin(cl); }
+  CRT_DI bool take(const DScene &, const Frame &, const Levels &, const uint32_t i, Ray &ray, uint32_t &) const {
+    query_ray(qb.rays, i, ray);
+    return true;
+  }
+  CRT_DI void begin(const Ray &, const uint32_t i, uint32_t &id) {
+    closest_begin(cl);
+    id = i;
+  }
+  CRT_DI float tri_dist() const { return 0.f; }
+  CRT_DI float limit() const { return cl.min_t; }
+  CRT_DI bool allow_behind() const { return cl.min_t < CRT_INF; }
+  template <bool COUNT>
+  CRT_DI bool tri(const DScene &s, WarpShare &ws, const bool parked, const bool flush, Trav &tv, uint32_t &n_tris) {
+    bool dummy = false;
+    tri_phase<false, PRIMARY, COUNT>(s, ws, parked, flush, tv.tref, tv.tend, cl, dummy, n_tris);
+    return false;
+  }
+  CRT_DI void answer(const Levels &, const uint32_t i) const { query_store_hit(sc, qb.hits, i, cl.best_tri, cl.best_t); }
+  CRT_DI bool handoff(const Levels &lv, const bool want, const uint32_t i, const Trav &tv, bool &closed) const {
+    return tail_handoff(lv, 0u, want, i, tv, cl.best_t, cl.best_tri, closed);
+  }
+  CRT_DI void finish(const Levels &) const {}
+};
+
+// Any hit of ray i within max_distance[i]: occluded iff some candidate has |P - o| <= max_distance (refractive meshes
+// skipped, AccelerationStructure.cpp:67-74).  A query has no light term, so no walk is skipped for a zero term.
+struct QueryShadowWalk {
+  static constexpr bool PRIMARY = false, SHADOW = true;
+  static constexpr uint32_t STAT_NODES = CRT_STAT_NODES_SHADOW, STAT_TRIS = CRT_STAT_TRIS_SHADOW;
+  const QueryBatch &qb;
+  const uint32_t total;
+  float dist = 0.0f, t_limit = 0.0f;
+  bool occluded = false;
+  CRT_DI explicit QueryShadowWalk(const QueryBatch &b) : qb(b), total(b.n) {}
+  CRT_DI bool take(const DScene &, const Frame &, const Levels &, const uint32_t i, Ray &ray, uint32_t &) {
+    query_ray(qb.rays, i, ray);
+    dist = qb.max_distance[i];
+    return true;
+  }
+  CRT_DI void begin(const Ray &ray, const uint32_t i, uint32_t &id) {
+    t_limit = query_shadow_limit(ray, dist);
+    occluded = false;
+    id = i;
+  }
+  CRT_DI float tri_dist() const { return dist; }
+  CRT_DI float limit() const { return t_limit; }
+  CRT_DI bool allow_behind() const { return true; }
+  template <bool COUNT>
+  CRT_DI bool tri(const DScene &sc, WarpShare &ws, const bool parked, const bool flush, Trav &tv, uint32_t &n_tris) {
+    Closest unused;
+    tri_phase<true, false, COUNT>(sc, ws, parked, flush, tv.tref, tv.tend, unused, occluded, n_tris);
+    return occluded;
+  }
+  CRT_DI void answer(const Levels &, const uint32_t i) const { qb.occluded[i] = occluded ? 1 : 0; }
+  CRT_DI bool handoff(const Levels &lv, const bool want, const uint32_t i, const Trav &tv, bool &closed) const {
+    return tail_handoff(lv, CRT_MAX_LEVELS, want, i, tv, 0.0f, CRT_INVALID, closed);
+  }
+  CRT_DI void finish(const Levels &) const {}
+};
+
+// lv: the query's own Levels (stats, hand-off records and counters; no ray queues).  Flags as k_closest / k_shadow's.
+template <bool PRIMARY, bool COUNT, int REFILL, bool CULL, bool WIDE>
+__global__ void __launch_bounds__(CRT_TRAV_BLOCK, CRT_TRAV_MIN_BLOCKS) k_query_closest(const DScene sc, const Levels lv, const QueryBatch qb,
+                                                                                    uint32_t *__restrict__ work_counter) {
+  __shared__ WarpShare s_ws[CRT_TRAV_BLOCK / 32];
+  WarpShare &ws = s_ws[threadIdx.x >> 5];
+  const Frame fr{};
+  QueryClosestWalk<PRIMARY> w(sc, qb);
+  walk_loop<REFILL, CULL, WIDE, false, (COUNT ? 0 : (WIDE ? 2 : 1)), COUNT, !COUNT, false>(sc, fr, lv, work_counter, ws, w);
+}
+
+template <int COUNT, int REFILL, bool CULL, bool WIDE>
+__global__ void __launch_bounds__(CRT_TRAV_BLOCK, CRT_TRAV_MIN_BLOCKS) k_query_shadow(const DScene sc, const Levels lv, const QueryBatch qb,
+                                                                                   uint32_t *__restrict__ work_counter) {
+  __shared__ WarpShare s_ws[CRT_TRAV_BLOCK / 32];
+  WarpShare &ws = s_ws[threadIdx.x >> 5];
+  const Frame fr{};
+  QueryShadowWalk w(qb);
+  walk_loop<REFILL, CULL, WIDE, true, (COUNT == 1 ? 0 : (WIDE ? 2 : 1)), (COUNT != 0), COUNT == 0, COUNT != 1>(
+      sc, fr, lv, work_counter, ws, w);
+}
+
+// The ray source of k_coop_query: record id = ray id of the batch
+struct CoopQuerySrc {
+  const QueryBatch &qb;
+  template <bool SHADOW, bool PRIMARY>
+  CRT_DI void ray(const DScene &, const Levels &, const uint32_t id, Ray &ray, float &dist) const {
+    query_ray(qb.rays, id, ray);
+    if (SHADOW) dist = qb.max_distance[id];
+  }
+  CRT_DI float shadow_limit(const Ray &ray, const float dist) const { return query_shadow_limit(ray, dist); }
+  CRT_DI void shadow_answer(const Levels &, const uint32_t id, const bool occluded) const { qb.occluded[id] = occluded ? 1 : 0; }
+  CRT_DI void closest_answer(const DScene &sc, const Levels &, const uint32_t id, const Closest &cl) const {
+    query_store_hit(sc, qb.hits, id, cl.best_tri, cl.best_t);
+  }
+};
+
+// k_coop over the walks a query kernel handed off.  Hand-off implies culling (crtb200_trace_rays_device), so CULL = true.
+template <bool SHADOW, bool PRIMARY>
+__global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_coop_query(const DScene sc, const Levels lv, const QueryBatch qb,
+                                                                                       const uint32_t early) {
+  __shared__ WarpCoop s_wc[CRT_COOP_WARPS];
+  coop_walks<SHADOW, PRIMARY, true, CRT_COOP_GROUP, true>(sc, lv, 0u, early, s_wc[threadIdx.x >> 5], CoopQuerySrc{qb});
 }
 
 }  // namespace crtd

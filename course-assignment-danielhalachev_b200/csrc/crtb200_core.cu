@@ -229,6 +229,18 @@ struct crtb200_ctx {
     }
   };
   std::vector<QueueSet> sets;
+  // caller-supplied ray batches (crtb200_trace_rays_device, DESIGN.md 3.12): the query's own scratch on this GPU, a
+  // QueueSet without ray queues (work cursors and hand-off counters in ctl, hand-off records in ovf, the early k_coop
+  // pass's side stream; `stream` is the caller's during a query), its device counters and grid sizes; on the first GPU
+  // of the context also the last query's span, GPU count and statistics
+  QueueSet query;
+  DevBuf<unsigned long long> query_stats_dev;
+  int blocks_query_closest = 0, blocks_query_shadow = 0;
+  bool query_ready = false;  // every part of the query scratch exists (set last by query_scratch)
+  cudaEvent_t query_ev[2] = {nullptr, nullptr};
+  uint32_t query_gpus = 0;
+  bool query_pending = false;
+  crtb200_stats query_last{};
   uint32_t concurrency = 2;  // chunk streams of a host-bound frame (tools/e2e_time.py, run r2aq: 2 streams with one chunk each
                              // at 1080p, two each at 4K; 4 streams x 2 chunks cost 1080p frames 15-17 %)
   cudaEvent_t fork_ev = nullptr;
@@ -443,6 +455,13 @@ int crtb200_destroy(crtb200_ctx *c) {
     if (q.coop_fork) cudaEventDestroy(q.coop_fork);
     if (q.coop_join) cudaEventDestroy(q.coop_join);
   }
+  c->query.release();  // (query.stream is the last caller's, not the context's)
+  if (c->query.coop_stream) cudaStreamDestroy(c->query.coop_stream);
+  if (c->query.coop_fork) cudaEventDestroy(c->query.coop_fork);
+  if (c->query.coop_join) cudaEventDestroy(c->query.coop_join);
+  c->query_stats_dev.release();
+  for (auto &e : c->query_ev)
+    if (e) cudaEventDestroy(e);
   if (c->band_stream) cudaStreamDestroy(c->band_stream);
   if (c->band_done) cudaEventDestroy(c->band_done);
   for (cudaEvent_t e : c->chunk_done) cudaEventDestroy(e);
@@ -1456,6 +1475,18 @@ static cudaEvent_t next_event(crtb200_ctx *c) {
 // dynamic shared memory of the kernels that walk one ray per lane: the visited-mesh bitset of scenes with > 64 meshes
 static size_t dyn_smem(const crtb200_ctx *c, int block) { return (size_t)c->sc.dedup_words * (size_t)block * sizeof(uint32_t); }
 
+// A caller's device pointer: device memory of the context's first GPU, `align`-byte aligned
+static int check_device_ptr(const crtb200_ctx *c, const void *p, size_t align, const char *what) {
+  if (!p) return fail(CRTB200_ERR_ARG, std::string(what) + " is null");
+  if (reinterpret_cast<uintptr_t>(p) % align) return fail(CRTB200_ERR_ARG, std::string(what) + " is not " + std::to_string(align) + "-byte aligned");
+  cudaPointerAttributes a{};
+  const cudaError_t e = cudaPointerGetAttributes(&a, p);
+  if (e != cudaSuccess) cudaGetLastError();  // (not a CUDA pointer: not sticky)
+  if (e != cudaSuccess || a.type != cudaMemoryTypeDevice || a.device != c->device)
+    return fail(CRTB200_ERR_ARG, std::string(what) + " is not device memory of the context's first GPU");
+  return CRTB200_OK;
+}
+
 // The kernel flavours of one frame.  traversal 0 (default): conservative culling + tail hand-off, both exact and both
 // resting on the nesting property of the uploaded trees; traversal 1 and the visit-all counting mode walk the
 // reference's literal itinerary.  The WIDE flavour (visited-mesh set in shared memory) only for scenes that need it, and
@@ -1473,6 +1504,17 @@ static Flavour frame_flavour(const crtb200_ctx *c, const crtb200_options *o) {
                  c->sampling.use_gi != 0,
                  o->count_work == 0 && wide,
                  o->count_work != 1 && wide};
+}
+
+// The kernel flavours of a caller's ray batch (crtb200_trace_rays_device): a frame's with the batch's traversal and
+// count_work -- literal walk without hand-off for traversal 1, count_work 1 and trees that do not nest -- never GI.
+static Flavour query_flavour(const crtb200_ctx *c, const crtb200_ray_batch *b) {
+  crtb200_options o{};
+  o.traversal = b->traversal;
+  o.count_work = b->count_work;
+  Flavour fl = frame_flavour(c, &o);
+  fl.gi = false;
+  return fl;
 }
 
 // f(v) with v as a compile-time constant: how the launch functions below turn a Flavour into template arguments
@@ -1514,42 +1556,130 @@ static void launch_coop(crtb200_ctx *c, const Flavour &fl, const Frame &fr, crtb
     }); }); }); });
 }
 
-// One traversal launch -- k_closest of level `level`, or the shadow pass -- and with hand-off k_coop around it (DESIGN.md
-// 3.8).  With an early pass (one queue set, not on a secondary level) the side stream is forked BEFORE the traversal
-// kernel is launched; behind it k_mark marks the traversal kernel's end, the early pass starts on the side stream (its
-// blocks get SM resources as the traversal kernel's blocks exit) and joins, and the final pass runs over what is left.
+// One traversal launch -- k_closest of level `level`, the shadow pass, or a query kernel -- and with hand-off k_coop
+// around it (DESIGN.md 3.8).  launch(stream, coop_blocks, early) enqueues the walk source's traversal kernel
+// (coop_blocks = 0) or its k_coop pass.  With an early pass (`early_ok`: one queue set, and not a secondary level of a
+// frame) the side stream is forked BEFORE the traversal kernel is launched; behind it k_mark marks the traversal kernel's
+// end, the early pass starts on the side stream (its blocks get SM resources as the traversal kernel's blocks exit)
+// and joins, and the final pass runs over what is left.
 // per_kernel: time them (closest_ms, shadow_ms, coop_*_ms); a mark with a kind (0 closest, 1 shadow, 2 / 3 their k_coop
 // part) opens a span and the next mark closes it, collect_stats_one reads them in pairs.
-static int traverse(crtb200_ctx *c, const Flavour &fl, const Frame &fr, crtb200_ctx::QueueSet &q, bool shadow, uint32_t level,
-                    bool per_kernel, uint32_t &launches) {
+template <typename Launch>
+static int traverse(crtb200_ctx *c, bool handoff, bool early_ok, crtb200_ctx::QueueSet &q, bool shadow, uint32_t level,
+                    bool per_kernel, uint32_t &launches, const Launch &launch) {
   auto mark = [&](int kind) {
     if (per_kernel) cudaEventRecord(next_event(c), q.stream);
     if (per_kernel && kind >= 0) c->kev_kind.push_back(kind);
   };
-  const bool early = fl.handoff && c->coop_early > 0 && c->cap_sets == 1 && (shadow || level == 0);
+  const bool early = handoff && c->coop_early > 0 && early_ok;
   mark(shadow ? 1 : 0);
   if (early) {
     CUDA_TRY(cudaEventRecord(q.coop_fork, q.stream));
     CUDA_TRY(cudaStreamWaitEvent(q.coop_stream, q.coop_fork, 0));
   }
-  if (shadow)
-    launch_shadow(c, fl, fr, q);
-  else
-    launch_closest(c, fl, fr, q, level);
-  if (fl.handoff) {
+  launch(q.stream, 0, 0u);
+  if (handoff) {
     mark(-1);
     mark(shadow ? 3 : 2);
     if (early) {
       k_mark<<<1, 32, 0, q.stream>>>(q.lv.ovf_ctl + CRT_CTL_STRIDE * (shadow ? (uint32_t)CRT_MAX_LEVELS : level) + 24u);
-      launch_coop(c, fl, fr, q, shadow, level, c->sm_count * c->coop_early, q.coop_stream, 1u);
+      launch(q.coop_stream, c->sm_count * c->coop_early, 1u);
       CUDA_TRY(cudaEventRecord(q.coop_join, q.coop_stream));
       CUDA_TRY(cudaStreamWaitEvent(q.stream, q.coop_join, 0));
       launches += 2;
     }
-    launch_coop(c, fl, fr, q, shadow, level, c->blocks_coop, q.stream, 0u);
+    launch(q.stream, c->blocks_coop, 0u);
     launches++;
   }
   mark(-1);
+  return CRTB200_OK;
+}
+
+// traverse for k_closest of level `level` or the shadow pass of a frame's chunk
+static int traverse_frame(crtb200_ctx *c, const Flavour &fl, const Frame &fr, crtb200_ctx::QueueSet &q, bool shadow, uint32_t level,
+                          bool per_kernel, uint32_t &launches) {
+  return traverse(c, fl.handoff, c->cap_sets == 1 && (shadow || level == 0), q, shadow, level, per_kernel, launches,
+                  [&](cudaStream_t st, int coop_blocks, uint32_t early) {
+                    if (coop_blocks)
+                      launch_coop(c, fl, fr, q, shadow, level, coop_blocks, st, early);
+                    else if (shadow)
+                      launch_shadow(c, fl, fr, q);
+                    else
+                      launch_closest(c, fl, fr, q, level);
+                  });
+}
+
+// One query batch `qb` on GPU x (its range of a multi-GPU batch) on stream st: the query's counters zeroed, the query
+// kernel of the ray type and, with hand-off, k_coop_query around it (traverse).  Closest hits use the work cursor and
+// hand-off line of launch 0, shadow queries those of launch CRT_MAX_LEVELS, as k_coop_query reads them.
+static int enqueue_query(crtb200_ctx *x, const Flavour &fl, uint32_t ray_type, const QueryBatch &qb, cudaStream_t st,
+                         uint32_t &launches) {
+  crtb200_ctx::QueueSet &q = x->query;
+  q.stream = st;
+  q.lv.tail_iters = fl.handoff ? (uint32_t)(x->tail_iters + 1) : 0u;
+  q.lv.tail_start = (uint32_t)x->tail_start;
+  q.lv.tail_start_closest = (uint32_t)x->tail_start_closest;
+  q.lv.tail_small = (uint32_t)x->tail_small;
+  CUDA_TRY(cudaMemsetAsync(q.ctl.p, 0, q.ctl.n * sizeof(uint32_t), st));
+  CUDA_TRY(cudaMemsetAsync(x->query_stats_dev.p, 0, CRT_STAT_SLOTS * sizeof(unsigned long long), st));
+  const bool shadow = ray_type == CRTB200_RAY_SHADOW, primary = ray_type == CRTB200_RAY_PRIMARY;
+  uint32_t *const work = q.work + CRT_CTL_STRIDE * (shadow ? (uint32_t)CRT_MAX_LEVELS : 0u);
+  launches++;
+  return traverse(x, fl.handoff, true, q, shadow, 0, false, launches, [&](cudaStream_t s, int coop_blocks, uint32_t early) {
+    if (coop_blocks) {
+      as_const(shadow, [&](auto sh) { as_const(primary, [&](auto prim) {
+        if constexpr (!(sh && prim)) k_coop_query<sh, prim><<<coop_blocks, 32 * CRT_COOP_WARPS, 0, s>>>(x->sc, q.lv, qb, early);
+      }); });
+    } else if (shadow) {
+      as_const_count(fl.count_work, [&](auto count) { as_const(fl.cull, [&](auto cull) { as_const(fl.wide_shadow, [&](auto wide) {
+        if constexpr (count != 1 || !(cull || wide))
+          k_query_shadow<count, CRT_REFILL_SHADOW, cull, wide>
+              <<<x->blocks_query_shadow, CRT_TRAV_BLOCK, wide ? dyn_smem(x, CRT_TRAV_BLOCK) : 0, s>>>(x->sc, q.lv, qb, work);
+      }); }); });
+    } else {
+      as_const(fl.count_work != 0, [&](auto count) { as_const(fl.cull, [&](auto cull) { as_const(fl.wide_closest, [&](auto wide) {
+        as_const(primary, [&](auto prim) {
+          if constexpr (!(count && wide))
+            k_query_closest<prim, count, CRT_REFILL_CLOSEST, cull, wide>
+                <<<x->blocks_query_closest, CRT_TRAV_BLOCK, dyn_smem(x, CRT_TRAV_BLOCK), s>>>(x->sc, q.lv, qb, work);
+        }); }); }); });
+    }
+  });
+}
+
+// The query scratch of GPU x, allocated on first use: work cursors | hand-off counters (ctl, the layout of a frame's
+// queue set), hand-off records for every lane of a query grid up to k_coop's capacity (ovf, all "not published"),
+// device counters, the early pass's side stream, and the span events of the first GPU.
+static int query_scratch(crtb200_ctx *x) {
+  crtb200_ctx::QueueSet &q = x->query;
+  if (x->query_ready) return CRTB200_OK;
+  int occ = 0;
+  CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_query_closest<true, false, CRT_REFILL_CLOSEST, true, false>, CRT_TRAV_BLOCK, 0));
+  x->blocks_query_closest = std::max(1, occ) * x->sm_count;
+  CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_query_shadow<0, CRT_REFILL_SHADOW, true, false>, CRT_TRAV_BLOCK, 0));
+  x->blocks_query_shadow = std::max(1, occ) * x->sm_count;
+  const uint64_t lanes = (uint64_t)std::max(x->blocks_query_closest, x->blocks_query_shadow) * CRT_TRAV_BLOCK;
+  const uint64_t cap = std::min<uint64_t>(lanes, (uint64_t)x->tail_cap * x->blocks_coop * CRT_COOP_WARPS);
+  CUDA_TRY(q.ovf.ensure(3 * cap));
+  CUDA_TRY(cudaMemset(q.ovf.p, 0xFF, 3 * cap * sizeof(uint4)));
+  CUDA_TRY(cudaStreamSynchronize(nullptr));  // (the query runs on the caller's stream, which may not wait for stream 0)
+  const size_t n_work = CRT_CTL_STRIDE * (CRT_MAX_LEVELS + 2), n_ovf = CRT_CTL_STRIDE * (CRT_MAX_LEVELS + 1);
+  CUDA_TRY(q.ctl.ensure(n_work + n_ovf));
+  CUDA_TRY(x->query_stats_dev.ensure(CRT_STAT_SLOTS));
+  int lo = 0, hi = 0;
+  CUDA_TRY(cudaDeviceGetStreamPriorityRange(&lo, &hi));
+  // (each part is created once: a call that failed half-way is completed by the next one)
+  if (!q.coop_stream) CUDA_TRY(cudaStreamCreateWithPriority(&q.coop_stream, cudaStreamNonBlocking, lo));
+  if (!q.coop_fork) CUDA_TRY(cudaEventCreateWithFlags(&q.coop_fork, cudaEventDisableTiming));
+  if (!q.coop_join) CUDA_TRY(cudaEventCreateWithFlags(&q.coop_join, cudaEventDisableTiming));
+  for (auto &e : x->query_ev)
+    if (!e) CUDA_TRY(cudaEventCreate(&e));
+  q.work = q.ctl.p;
+  q.lv.ovf = q.ovf.p;
+  q.lv.ovf_ctl = q.ctl.p + n_work;
+  q.lv.ovf_cap = (uint32_t)cap;
+  q.lv.stats = x->query_stats_dev.p;
+  x->query_ready = true;
   return CRTB200_OK;
 }
 
@@ -1623,12 +1753,12 @@ static int sample_pass(crtb200_ctx *c, const FrameReq &r, const Flavour &fl, Fra
   q.lv.tail_start_closest = (uint32_t)c->tail_start_closest;
   q.lv.tail_small = (uint32_t)c->tail_small;
   for (uint32_t l = 0; l < levels; l++) {
-    const int rc = traverse(c, fl, fr, q, false, l, per_kernel, launches);
+    const int rc = traverse_frame(c, fl, fr, q, false, l, per_kernel, launches);
     if (rc) return rc;
     as_const(fl.gi, [&](auto gi) { k_shade<gi><<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, l); });
     launches += 2;
   }
-  const int rc = traverse(c, fl, fr, q, true, 0, per_kernel, launches);
+  const int rc = traverse_frame(c, fl, fr, q, true, 0, per_kernel, launches);
   if (rc) return rc;
   k_accumulate<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv);
   launches += 2;
@@ -2488,23 +2618,36 @@ int crtb200_assemble_shards(crtb200_ctx *c, const float *d_slabs, uint32_t shard
   return CRTB200_OK;
 }
 
+int crtb200_generate_rays_device(crtb200_ctx *c, const crtb200_camera *cam, float *d_rays_out, void *stream) {
+  ErrScope scope(c);
+  if (!c || !cam) return fail(CRTB200_ERR_ARG, "null argument");
+  if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
+  CUDA_TRY(cudaSetDevice(c->device));
+  int rc = check_device_ptr(c, d_rays_out, 4, "d_rays_out");
+  if (rc) return rc;
+  DCamera dc;
+  for (int k = 0; k < 3; k++) dc.pos[k] = cam->position[k];
+  for (int k = 0; k < 9; k++) dc.rot[k] = cam->rotation[k];
+  k_generate_rays<<<c->sm_count * 8, 256, 0, (cudaStream_t)stream>>>(c->sc, dc, d_rays_out);
+  CUDA_TRY(cudaGetLastError());
+  return CRTB200_OK;
+}
+
 int crtb200_generate_rays(crtb200_ctx *c, const crtb200_camera *cam, float *rays_out) {
   ErrScope scope(c);
   if (!c || !cam || !rays_out) return fail(CRTB200_ERR_ARG, "null argument");
   if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
   CUDA_TRY(cudaSetDevice(c->device));
   const size_t n = (size_t)c->sc.width * c->sc.height;
+  if (n == 0) return CRTB200_OK;
   DevBuf<float> d;
   CUDA_TRY(d.ensure(n * 6));
-  DCamera dc;
-  for (int k = 0; k < 3; k++) dc.pos[k] = cam->position[k];
-  for (int k = 0; k < 9; k++) dc.rot[k] = cam->rotation[k];
-  k_generate_rays<<<c->sm_count * 8, 256, 0, c->stream>>>(c->sc, dc, d.p);
-  cudaError_t e = cudaMemcpyAsync(rays_out, d.p, n * 6 * sizeof(float), cudaMemcpyDeviceToHost, c->stream);
+  int rc = crtb200_generate_rays_device(c, cam, d.p, c->stream);
+  cudaError_t e = rc ? cudaSuccess : cudaMemcpyAsync(rays_out, d.p, n * 6 * sizeof(float), cudaMemcpyDeviceToHost, c->stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
   d.release();
   CUDA_TRY(e);
-  return CRTB200_OK;
+  return rc;
 }
 
 int crtb200_scene_trees(crtb200_ctx *c, crtb200_trees *t) {
@@ -2586,22 +2729,118 @@ int crtb200_debug_powf5(crtb200_ctx *c, const float *x, uint32_t n, float *out) 
   return CRTB200_OK;
 }
 
+// the checks of a ray batch that need no pointer attributes (crtb200_trace_rays_device and its host wrapper)
+static int check_batch(crtb200_ctx *c, const crtb200_ray_batch *b) {
+  if (!c || !b || !b->rays) return fail(CRTB200_ERR_ARG, "null argument");
+  if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
+  if (b->n >= 0x80000000u) return fail(CRTB200_ERR_ARG, "a ray batch holds fewer than 2^31 rays");
+  if (b->ray_type > CRTB200_RAY_REFRACTION) return fail(CRTB200_ERR_ARG, "bad ray type (primary, shadow, reflection or refraction)");
+  if (b->traversal > 1) return fail(CRTB200_ERR_ARG, "unknown traversal mode");
+  if (b->count_work > 2) return fail(CRTB200_ERR_ARG, "unknown count_work mode");
+  if (b->ray_type == CRTB200_RAY_SHADOW ? (!b->max_distance || !b->occluded) : !b->hits)
+    return fail(CRTB200_ERR_ARG, "missing output / distance array");
+  return CRTB200_OK;
+}
+
+int crtb200_trace_rays_device(crtb200_ctx *c, const crtb200_ray_batch *b, void *stream) {
+  ErrScope scope(c);
+  int rc = check_batch(c, b);
+  if (rc || b->n == 0) return rc;
+  CUDA_TRY(cudaSetDevice(c->device));
+  const bool shadow = b->ray_type == CRTB200_RAY_SHADOW;
+  if ((rc = check_device_ptr(c, b->rays, 4, "rays"))) return rc;
+  if (shadow && ((rc = check_device_ptr(c, b->max_distance, 4, "max_distance")) || (rc = check_device_ptr(c, b->occluded, 1, "occluded"))))
+    return rc;
+  if (!shadow && (rc = check_device_ptr(c, b->hits, 4, "hits"))) return rc;
+  static_assert(sizeof(HitRec) == sizeof(crtb200_hit), "hit records are written in the public layout");
+  // contiguous ranges, one per GPU (a batch smaller than the GPU list uses its first n GPUs)
+  const std::vector<crtb200_ctx *> all = all_gpus(c);
+  const uint32_t g = (uint32_t)std::min<size_t>(all.size(), b->n);
+  for (uint32_t i = 0; i < g; i++) {
+    CUDA_TRY(cudaSetDevice(all[i]->device));
+    if ((rc = query_scratch(all[i]))) return rc;
+  }
+  CUDA_TRY(cudaSetDevice(c->device));
+  const cudaStream_t st = (cudaStream_t)stream;
+  const Flavour fl = query_flavour(c, b);
+  c->query_pending = false;
+  CUDA_TRY(cudaEventRecord(c->query_ev[0], st));
+  if (g > 1) CUDA_TRY(cudaEventRecord(c->multi_fork, st));
+  uint32_t launches = 0, forked = 0;
+  for (uint32_t i = 0; i < g && rc == CRTB200_OK; i++) {
+    crtb200_ctx *x = all[i];
+    const uint64_t begin = (uint64_t)b->n * i / g, end = (uint64_t)b->n * (i + 1) / g;
+    const QueryBatch qb{b->rays + 6 * begin, shadow ? b->max_distance + begin : nullptr,
+                        shadow ? nullptr : reinterpret_cast<HitRec *>(b->hits + begin), shadow ? b->occluded + begin : nullptr,
+                        (uint32_t)(end - begin)};
+    CUDA_TRY(cudaSetDevice(x->device));
+    const cudaStream_t xs = i ? x->stream : st;
+    if (i) {
+      CUDA_TRY(cudaStreamWaitEvent(xs, c->multi_fork, 0));
+      forked = i;
+    }
+    rc = enqueue_query(x, fl, b->ray_type, qb, xs, launches);
+    if (rc == CRTB200_OK && cudaGetLastError() != cudaSuccess) rc = fail(CRTB200_ERR_CUDA, "a query launch failed");
+    // a peer is joined even when its part failed half-way: what it did enqueue writes into the caller's arrays
+    if (i && cudaEventRecord(x->multi_done, xs) != cudaSuccess && rc == CRTB200_OK) rc = fail(CRTB200_ERR_CUDA, "cudaEventRecord failed");
+  }
+  CUDA_TRY(cudaSetDevice(c->device));
+  for (uint32_t i = 1; i <= forked; i++) CUDA_TRY(cudaStreamWaitEvent(st, all[i]->multi_done, 0));
+  if (rc) return rc;
+  CUDA_TRY(cudaEventRecord(c->query_ev[1], st));
+  c->query_last = crtb200_stats{};
+  uint64_t *rays[4] = {&c->query_last.rays_primary, &c->query_last.rays_shadow, &c->query_last.rays_reflection,
+                       &c->query_last.rays_refraction};
+  *rays[b->ray_type] = b->n;
+  c->query_last.kernel_launches = launches;
+  c->query_gpus = g;
+  c->query_pending = true;
+  return CRTB200_OK;
+}
+
+int crtb200_last_query_stats(crtb200_ctx *c, crtb200_stats *stats) {
+  ErrScope scope(c);
+  if (!c || !stats) return fail(CRTB200_ERR_ARG, "null argument");
+  CUDA_TRY(cudaSetDevice(c->device));
+  if (c->query_pending) {
+    CUDA_TRY(cudaEventSynchronize(c->query_ev[1]));
+    float ms = 0.f;
+    CUDA_TRY(cudaEventElapsedTime(&ms, c->query_ev[0], c->query_ev[1]));
+    crtb200_stats &q = c->query_last;
+    q.device_ms = ms;
+    const std::vector<crtb200_ctx *> all = all_gpus(c);
+    for (uint32_t i = 0; i < c->query_gpus; i++) {
+      unsigned long long st[CRT_STAT_SLOTS];
+      CUDA_TRY(cudaSetDevice(all[i]->device));
+      CUDA_TRY(cudaMemcpy(st, all[i]->query_stats_dev.p, sizeof(st), cudaMemcpyDeviceToHost));
+      q.node_tests_closest += st[CRT_STAT_NODES_CLOSEST];
+      q.triangle_tests_closest += st[CRT_STAT_TRIS_CLOSEST];
+      q.node_tests_shadow += st[CRT_STAT_NODES_SHADOW];
+      q.triangle_tests_shadow += st[CRT_STAT_TRIS_SHADOW];
+      q.handoff_closest += st[CRT_STAT_HANDOFF_CLOSEST];
+      q.handoff_shadow += st[CRT_STAT_HANDOFF_SHADOW];
+    }
+    CUDA_TRY(cudaSetDevice(c->device));
+    c->query_pending = false;
+  }
+  *stats = c->query_last;
+  return CRTB200_OK;
+}
+
 int crtb200_trace_rays(crtb200_ctx *c, const float *rays, uint32_t n, uint32_t ray_type, uint32_t traversal,
                        const float *max_distance, crtb200_hit *hits_out, uint8_t *occluded_out) {
   ErrScope scope(c);
-  if (!c || !rays) return fail(CRTB200_ERR_ARG, "null argument");
-  if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
-  if (ray_type > 3) return fail(CRTB200_ERR_ARG, "bad ray type");
-  if (traversal > 1) return fail(CRTB200_ERR_ARG, "unknown traversal mode");  // caller-supplied rays always take the literal walk
-  if (ray_type == CRTB200_RAY_SHADOW ? (!max_distance || !occluded_out) : !hits_out) return fail(CRTB200_ERR_ARG, "missing output / distance array");
-  if (n == 0) return CRTB200_OK;
+  crtb200_ray_batch b{n, ray_type, traversal, 0, rays, max_distance, hits_out, occluded_out};
+  int rc = check_batch(c, &b);
+  if (rc || n == 0) return rc;
   CUDA_TRY(cudaSetDevice(c->device));
+  const bool shadow = ray_type == CRTB200_RAY_SHADOW;
   DevBuf<float> d_rays, d_dist;
-  DevBuf<HitRec> d_hits;
+  DevBuf<crtb200_hit> d_hits;
   DevBuf<uint8_t> d_occ;
   cudaError_t e = d_rays.ensure((size_t)n * 6);
   if (e == cudaSuccess) e = cudaMemcpyAsync(d_rays.p, rays, (size_t)n * 6 * sizeof(float), cudaMemcpyHostToDevice, c->stream);
-  if (ray_type == CRTB200_RAY_SHADOW) {
+  if (shadow) {
     if (e == cudaSuccess) e = d_dist.ensure(n);
     if (e == cudaSuccess) e = d_occ.ensure(n);
     if (e == cudaSuccess) e = cudaMemcpyAsync(d_dist.p, max_distance, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, c->stream);
@@ -2609,14 +2848,17 @@ int crtb200_trace_rays(crtb200_ctx *c, const float *rays, uint32_t n, uint32_t r
     e = d_hits.ensure(n);
   }
   if (e == cudaSuccess) {
-    k_query<<<c->sm_count * 8, 256, dyn_smem(c, 256), c->stream>>>(c->sc, d_rays.p, n, ray_type, d_dist.p, d_hits.p, d_occ.p);
-    e = cudaGetLastError();
+    b.rays = d_rays.p;
+    b.max_distance = d_dist.p;
+    b.hits = d_hits.p;
+    b.occluded = d_occ.p;
+    rc = crtb200_trace_rays_device(c, &b, c->stream);
   }
-  if (e == cudaSuccess) {
-    if (ray_type == CRTB200_RAY_SHADOW)
+  if (e == cudaSuccess && rc == CRTB200_OK) {
+    if (shadow)
       e = cudaMemcpyAsync(occluded_out, d_occ.p, n, cudaMemcpyDeviceToHost, c->stream);
     else
-      e = cudaMemcpyAsync(hits_out, d_hits.p, (size_t)n * sizeof(HitRec), cudaMemcpyDeviceToHost, c->stream);
+      e = cudaMemcpyAsync(hits_out, d_hits.p, (size_t)n * sizeof(crtb200_hit), cudaMemcpyDeviceToHost, c->stream);
   }
   if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
   d_rays.release();
@@ -2624,7 +2866,7 @@ int crtb200_trace_rays(crtb200_ctx *c, const float *rays, uint32_t n, uint32_t r
   d_hits.release();
   d_occ.release();
   CUDA_TRY(e);
-  return CRTB200_OK;
+  return rc;
 }
 
 }  // extern "C"

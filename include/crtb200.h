@@ -416,12 +416,52 @@ int crtb200_assemble_shards(crtb200_ctx *ctx, const float *d_slabs, uint32_t sha
                             uint8_t *d_rgb8_out, void *stream);
 
 /* replaces: RayTracer::getRay + the re-normalisation of shootRay (RayTracer.cpp:61-80,420), exposed so the
- * parity tests can compare primary rays bit for bit.  rays_out: H*W*6 float32 (origin xyz, direction xyz), host. */
+ * parity tests can compare primary rays bit for bit.  rays_out: H*W*6 float32 (origin xyz, direction xyz), host;
+ * crtb200_generate_rays_device copied back (synchronous). */
 int crtb200_generate_rays(crtb200_ctx *ctx, const crtb200_camera *camera, float *rays_out);
 
+/* replaces: RayTracer::getRay + the re-normalisation of shootRay (RayTracer.cpp:61-80,420) for every pixel, into caller
+ * DEVICE memory: d_rays_out holds H*W*6 float32 (layout of crtb200_generate_rays) on the context's first GPU, 4-byte
+ * aligned (else CRTB200_ERR_ARG; CRTB200_ERR_STATE without a scene).  Asynchronous on `stream` (a cudaStream_t, NULL = default), like
+ * crtb200_render_device: a camera-ray batch for crtb200_trace_rays_device without a host round trip. */
+int crtb200_generate_rays_device(crtb200_ctx *ctx, const crtb200_camera *camera, float *d_rays_out, void *stream);
+
+/* A batch of caller-supplied rays in DEVICE memory of the context's first GPU (DESIGN.md 3.12). */
+typedef struct crtb200_ray_batch {
+  uint32_t n;                /* rays; n < 2^31 (CRTB200_ERR_ARG otherwise); 0 = nothing to do                          */
+  uint32_t ray_type;         /* CRTB200_RAY_PRIMARY / _REFLECTION / _REFRACTION: closest hit; CRTB200_RAY_SHADOW: any hit */
+  uint32_t traversal;        /* as crtb200_options.traversal: 0 = culled walk + tail hand-off, 1 = the literal itinerary */
+  uint32_t count_work;       /* as crtb200_options.count_work (0 / 1 / 2)                                               */
+  const float *rays;         /* n * 6 float32: origin xyz, direction xyz (the crtb200_trace_rays layout)                */
+  const float *max_distance; /* n float32, shadow queries only                                                         */
+  crtb200_hit *hits;         /* n records, closest-hit queries only (public numbering; miss: -1, -1, t = 0)            */
+  uint8_t *occluded;         /* n bytes, shadow queries only                                                           */
+} crtb200_ray_batch;
+
+/* replaces: RayTracer::trace (RayTracer.cpp:453-458) and the non-GI RayTracer::hasIntersection (RayTracer.cpp:507-518)
+ * -- KDTree::intersect, public in the reference -- for caller-supplied rays held in device memory.  Closest hit follows
+ * RayTracer::trace, with the primary ray's back-face rule for CRTB200_RAY_PRIMARY only; a shadow query skips refractive
+ * meshes and answers 1 iff some candidate has |P - o| <= max_distance.  Directions need not be unit length; NaN,
+ * axis-parallel and zero directions behave as in the reference.  The answers do not depend on traversal, the GPU list or
+ * the stream.  The rays are walked by the production traversal loop, with culling and tail hand-off for traversal 0.
+ * On a crtb200_create_multi context the batch is split into contiguous ranges, one per GPU, each reading its rays and
+ * writing its answers in the first GPU's memory through the peer mapping.  Asynchronous on `stream` (a cudaStream_t,
+ * NULL = default), with the same rule about concurrent use of one context as crtb200_render_device.
+ * CRTB200_ERR_ARG: a pointer the ray type needs is not device memory of the context's first GPU, rays / max_distance /
+ * hits not 4-byte aligned, CRTB200_RAY_DIFFUSE or an unknown ray type, traversal or count_work, n >= 2^31.
+ * CRTB200_ERR_STATE without a scene.  A query never changes crtb200_last_stats, the sampling stats, the colour buffer or
+ * a progressive session; it keeps a small scratch per GPU, allocated on first use, until crtb200_destroy. */
+int crtb200_trace_rays_device(crtb200_ctx *ctx, const crtb200_ray_batch *batch, void *stream);
+/* replaces: nothing in the reference (it counts no rays).  After synchronisation: the last query's n in the rays_* field
+ * of its type, node and triangle tests under its count_work, handoff_*, device_ms (its span on the caller's stream)
+ * and kernel_launches, summed over the GPUs; every other field 0. */
+int crtb200_last_query_stats(crtb200_ctx *ctx, crtb200_stats *stats);
+
 /* replaces: RayTracer::trace (RayTracer.cpp:453-458) / RayTracer::hasIntersection (RayTracer.cpp:507-518) for caller-
- * supplied rays.  rays: n*6 float32 host; ray_type: CRTB200_RAY_*; for shadow queries max_distance holds n floats
- * and occluded_out n bytes; for closest-hit queries hits_out holds n records. */
+ * supplied rays in HOST memory: stages them to the device, runs crtb200_trace_rays_device on the context's stream and
+ * copies the answers back (synchronous).  rays: n*6 float32; ray_type: CRTB200_RAY_*; for shadow queries max_distance
+ * holds n floats and occluded_out n bytes; for closest-hit queries hits_out holds n records.  traversal as in
+ * crtb200_ray_batch (same answers either way). */
 int crtb200_trace_rays(crtb200_ctx *ctx, const float *rays, uint32_t n, uint32_t ray_type, uint32_t traversal,
                        const float *max_distance, crtb200_hit *hits_out, uint8_t *occluded_out);
 
