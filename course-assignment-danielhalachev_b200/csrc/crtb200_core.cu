@@ -104,15 +104,23 @@ struct Worker {
       return fail(CRTB200_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorName(e_) + ": " + cudaGetErrorString(e_)); \
   } while (0)
 
+// One device allocation, freed by its destructor; move-only.  Owners free on their own device: crtb200_destroy selects
+// the context's device before deleting it.
 template <typename T>
 struct DevBuf {
   T *p = nullptr;
   size_t n = 0;
+  DevBuf() = default;
+  DevBuf(DevBuf &&o) noexcept : p(std::exchange(o.p, nullptr)), n(std::exchange(o.n, 0)) {}
+  DevBuf &operator=(DevBuf o) noexcept {  // (o is moved in and frees what this held)
+    std::swap(p, o.p);
+    std::swap(n, o.n);
+    return *this;
+  }
+  ~DevBuf() { release(); }
   cudaError_t ensure(size_t count) {
     if (count <= n && p) return cudaSuccess;
-    if (p) cudaFree(p);
-    p = nullptr;
-    n = 0;
+    release();
     if (count == 0) return cudaSuccess;
     cudaError_t e = cudaMalloc(&p, count * sizeof(T));
     if (e == cudaSuccess) n = count;
@@ -131,16 +139,47 @@ struct DevBuf {
   }
 };
 
+// One CUDA stream or event, destroyed by its destructor; move-only, null until create() makes it.
+template <typename H>
+struct CudaHandle {
+  H h = nullptr;
+  CudaHandle() = default;
+  CudaHandle(CudaHandle &&o) noexcept : h(std::exchange(o.h, nullptr)) {}
+  CudaHandle &operator=(CudaHandle o) noexcept {
+    std::swap(h, o.h);
+    return *this;
+  }
+  ~CudaHandle() {
+    if (!h) return;
+    if constexpr (std::is_same_v<H, cudaStream_t>) cudaStreamDestroy(h);
+    else cudaEventDestroy(h);
+  }
+  operator H() const { return h; }
+  // Creates the handle unless it exists.  Streams: flags cudaStreamNonBlocking and `priority` (0 is the default
+  // priority); events: flags cudaEventDefault or cudaEventDisableTiming.
+  cudaError_t create(unsigned flags, int priority = 0) {
+    if (h) return cudaSuccess;
+    H x = nullptr;
+    cudaError_t e;
+    if constexpr (std::is_same_v<H, cudaStream_t>) e = cudaStreamCreateWithPriority(&x, flags, priority);
+    else e = cudaEventCreateWithFlags(&x, flags);
+    if (e == cudaSuccess) h = x;
+    return e;
+  }
+};
+using Stream = CudaHandle<cudaStream_t>;
+using Event = CudaHandle<cudaEvent_t>;
+
 // counters of a render kept beside crtb200_stats: diffuse rays, and an adaptive step's pixel-samples and stopped pixels
 struct SideCounts { uint64_t diffuse = 0, px_samples = 0, stopped = 0; };
 
 struct crtb200_ctx {
   int device = 0;
   int sm_count = 0;
-  cudaStream_t stream = nullptr;
-  cudaEvent_t ev[2] = {nullptr, nullptr};  // the last frame's span on the caller's stream
-  std::vector<cudaEvent_t> kev;  // per-launch event pairs: K2 / K3 timing
-  std::vector<int> kev_kind;     // 0 = closest, 1 = shadow, 2 / 3 their k_coop part (one entry per pair)
+  Stream stream;
+  Event ev[2];                // the last frame's span on the caller's stream
+  std::vector<Event> kev;     // per-launch event pairs: K2 / K3 timing
+  std::vector<int> kev_kind;  // 0 = closest, 1 = shadow, 2 / 3 their k_coop part (one entry per pair)
   size_t kev_used = 0;
   bool have_scene = false;
   uint64_t queue_budget = 16ull << 30;
@@ -195,8 +234,8 @@ struct crtb200_ctx {
   // frame f runs on copy_stream while frame f + 1 is rendered into the other pair
   DevBuf<float> frame_b;
   DevBuf<uint8_t> frame8_b;
-  cudaStream_t copy_stream = nullptr;
-  cudaEvent_t rendered[2] = {nullptr, nullptr}, copied[2] = {nullptr, nullptr};
+  Stream copy_stream;
+  Event rendered[2], copied[2];
   DevBuf<HitRec> hits;
   DevBuf<uint8_t> mask;
   std::vector<crtb200_rect> mask_rects;
@@ -217,33 +256,28 @@ struct crtb200_ctx {
     DevBuf<uint2> hit0;         //            ... and sample 0's primary hit
     DevBuf<uint32_t> alist, acount;  // adaptive passes: the chunk's active shard items and their count (k_adapt_compact)
     uint32_t *work = nullptr;   // into ctl
-    cudaStream_t stream = nullptr;
-    cudaEvent_t done = nullptr;
+    Stream stream;              // (frames only: a query runs on the caller's stream)
+    Event done;
     // early k_coop pass: low-priority side stream, forked before and joined behind every traversal launch
-    cudaStream_t coop_stream = nullptr;
-    cudaEvent_t coop_fork = nullptr, coop_join = nullptr;
-    void release() {
-      ray_o.release(); ray_d.release(); color.release(); dq.release(); hit_tri.release(); ctl.release();
-      hit_t.release(); comb.release(); vis.release(); ovf.release(); acc.release(); hit0.release();
-      alist.release(); acount.release();
-    }
+    Stream coop_stream;
+    Event coop_fork, coop_join;
   };
   std::vector<QueueSet> sets;
   // caller-supplied ray batches (crtb200_trace_rays_device, DESIGN.md 3.12): the query's own scratch on this GPU, a
-  // QueueSet without ray queues (work cursors and hand-off counters in ctl, hand-off records in ovf, the early k_coop
-  // pass's side stream; `stream` is the caller's during a query), its device counters and grid sizes; on the first GPU
-  // of the context also the last query's span, GPU count and statistics
+  // QueueSet without ray queues or stream (work cursors and hand-off counters in ctl, hand-off records in ovf, the
+  // early k_coop pass's side stream), its device counters and grid sizes; on the first GPU of the context also the
+  // last query's span, GPU count and statistics
   QueueSet query;
   DevBuf<unsigned long long> query_stats_dev;
   int blocks_query_closest = 0, blocks_query_shadow = 0;
   bool query_ready = false;  // every part of the query scratch exists (set last by query_scratch)
-  cudaEvent_t query_ev[2] = {nullptr, nullptr};
+  Event query_ev[2];
   uint32_t query_gpus = 0;
   bool query_pending = false;
   crtb200_stats query_last{};
   uint32_t concurrency = 2;  // chunk streams of a host-bound frame (tools/e2e_time.py, run r2aq: 2 streams with one chunk each
                              // at 1080p, two each at 4K; 4 streams x 2 chunks cost 1080p frames 15-17 %)
-  cudaEvent_t fork_ev = nullptr;
+  Event fork_ev;
   DevBuf<unsigned long long> stats_dev;
   uint32_t cap_items = 0;
   uint32_t cap_depth = 0xFFFFFFFFu;
@@ -254,10 +288,10 @@ struct crtb200_ctx {
   // the small secondary levels pay more for the extra launches and joins than they gain (hw11_room +2 %)
   int coop_early = CRT_COOP_MIN_BLOCKS;
   uint32_t n_chunks = 0;  // chunks of the current plan (chunk k runs on set k % cap_sets)
-  cudaStream_t band_stream = nullptr;  // device -> host band copies of a chunked host-bound frame
-  cudaEvent_t band_done = nullptr;
-  std::vector<cudaEvent_t> chunk_done;
-  std::vector<cudaEvent_t> dbg_ev;  // CRT_CHUNK_TIMES (tools): per chunk, end of k_store and end of its band copy
+  Stream band_stream;  // device -> host band copies of a chunked host-bound frame
+  Event band_done;
+  std::vector<Event> chunk_done;
+  std::vector<Event> dbg_ev;  // CRT_CHUNK_TIMES (tools): per chunk, end of k_store and end of its band copy
   uint32_t dbg_chunks = 0;
 
   int blocks_closest = 0, blocks_closest_sec = 0, blocks_shadow = 0, blocks_coop = 0;
@@ -295,8 +329,8 @@ struct crtb200_ctx {
   std::vector<std::unique_ptr<Worker>> workers;
   std::vector<int> worker_rc;
   std::vector<std::string> worker_msg;
-  cudaEvent_t multi_fork = nullptr;  // primary stream position the peers must wait for before touching the frame
-  cudaEvent_t multi_done = nullptr;  // (on a peer) its shard is stored
+  Event multi_fork;  // primary stream position the peers must wait for before touching the frame
+  Event multi_done;  // (on a peer) its shard is stored
   std::string error;                 // last error of a call on this context (crtb200_last_error_ctx)
 };
 static void note_ctx_error(crtb200_ctx *c, const std::string &msg) { c->error = msg; }
@@ -332,11 +366,11 @@ int crtb200_create(int device, crtb200_ctx **out) {
   crtb200_ctx *c = new crtb200_ctx();
   c->device = device;
   c->sm_count = prop.multiProcessorCount;
-  if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) {
+  if (c->stream.create(cudaStreamNonBlocking) != cudaSuccess || c->ev[0].create(cudaEventDefault) != cudaSuccess ||
+      c->ev[1].create(cudaEventDefault) != cudaSuccess) {
     delete c;
-    return fail(CRTB200_ERR_CUDA, "cudaStreamCreate failed");
+    return fail(CRTB200_ERR_CUDA, "cudaStreamCreate / cudaEventCreate failed");
   }
-  for (auto &e : c->ev) cudaEventCreate(&e);
   int occ = 0;
   cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_closest<true, false, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, false, false>, CRT_TRAV_BLOCK, 0);
   c->blocks_closest = std::max(1, occ) * c->sm_count;
@@ -395,7 +429,7 @@ int crtb200_create_multi(const int *device_ids, int n, crtb200_ctx **out) {
         rc = fail(CRTB200_ERR_CUDA, std::string("peer access from device ") + std::to_string(p->device) + " to device " +
                                         std::to_string(c->device) + ": " + cudaGetErrorString(e));
     }
-    if (rc == CRTB200_OK && cudaEventCreateWithFlags(&p->multi_done, cudaEventDisableTiming) != cudaSuccess)
+    if (rc == CRTB200_OK && p->multi_done.create(cudaEventDisableTiming) != cudaSuccess)
       rc = fail(CRTB200_ERR_CUDA, "cudaEventCreate failed");
     if (rc) {
       if (p) crtb200_destroy(p);
@@ -408,7 +442,7 @@ int crtb200_create_multi(const int *device_ids, int n, crtb200_ctx **out) {
   c->worker_rc.assign(c->peers.size(), 0);
   c->worker_msg.assign(c->peers.size(), std::string());
   cudaSetDevice(c->device);
-  if (!c->peers.empty() && cudaEventCreateWithFlags(&c->multi_fork, cudaEventDisableTiming) != cudaSuccess) {
+  if (!c->peers.empty() && c->multi_fork.create(cudaEventDisableTiming) != cudaSuccess) {
     crtb200_destroy(c);
     return fail(CRTB200_ERR_CUDA, "cudaEventCreate failed");
   }
@@ -427,50 +461,9 @@ int crtb200_device_list(const crtb200_ctx *c, int *device_ids, int capacity, int
 int crtb200_destroy(crtb200_ctx *c) {
   if (!c) return CRTB200_OK;
   c->workers.clear();  // joins the helper threads
-  for (crtb200_ctx *p : c->peers) crtb200_destroy(p);
-  c->peers.clear();
-  cudaSetDevice(c->device);
+  for (crtb200_ctx *p : c->peers) crtb200_destroy(p);  // first: their kernels store into this context's memory
+  cudaSetDevice(c->device);  // the members free their buffers, streams and events on this device
   cudaStreamSynchronize(c->stream);
-  if (c->multi_fork) cudaEventDestroy(c->multi_fork);
-  if (c->multi_done) cudaEventDestroy(c->multi_done);
-  c->arena.release(); c->vtx_normal.release(); c->top_refs.release();
-  c->tri_shade.release(); c->vtx_uv.release(); c->meshes.release(); c->materials.release(); c->textures.release();
-  c->texels.release(); c->lights.release(); c->frame.release(); c->frame8.release(); c->hits.release();
-  c->mask.release(); c->frame_b.release(); c->frame8_b.release();
-  c->acc_sum.release(); c->acc_sumsq.release(); c->acc_hit.release();
-  c->kd_nodes.release(); c->kd_refs.release();
-  if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
-  for (int k = 0; k < 2; k++) {
-    if (c->rendered[k]) cudaEventDestroy(c->rendered[k]);
-    if (c->copied[k]) cudaEventDestroy(c->copied[k]);
-  }
-  for (auto &q : c->sets) {
-    q.release();
-    if (q.stream) cudaStreamDestroy(q.stream);
-    if (q.done) cudaEventDestroy(q.done);
-  }
-  if (c->fork_ev) cudaEventDestroy(c->fork_ev);
-  for (auto &q : c->sets) {
-    if (q.coop_stream) cudaStreamDestroy(q.coop_stream);
-    if (q.coop_fork) cudaEventDestroy(q.coop_fork);
-    if (q.coop_join) cudaEventDestroy(q.coop_join);
-  }
-  c->query.release();  // (query.stream is the last caller's, not the context's)
-  if (c->query.coop_stream) cudaStreamDestroy(c->query.coop_stream);
-  if (c->query.coop_fork) cudaEventDestroy(c->query.coop_fork);
-  if (c->query.coop_join) cudaEventDestroy(c->query.coop_join);
-  c->query_stats_dev.release();
-  for (auto &e : c->query_ev)
-    if (e) cudaEventDestroy(e);
-  if (c->band_stream) cudaStreamDestroy(c->band_stream);
-  if (c->band_done) cudaEventDestroy(c->band_done);
-  for (cudaEvent_t e : c->chunk_done) cudaEventDestroy(e);
-  for (cudaEvent_t e : c->dbg_ev) cudaEventDestroy(e);
-  c->stats_dev.release();
-  for (auto &e : c->ev)
-    if (e) cudaEventDestroy(e);
-  for (auto &e : c->kev) cudaEventDestroy(e);
-  if (c->stream) cudaStreamDestroy(c->stream);
   delete c;
   return CRTB200_OK;
 }
@@ -1099,19 +1092,9 @@ static int upload_geometry_one(crtb200_ctx *c, const crtb200_scene *s, bool keep
   alloc_level(lv[0], T);
   if (!ok) return nomem();
 
-  cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-  CUDA_TRY(cudaEventCreate(&ev0));
-  if (cudaEventCreate(&ev1) != cudaSuccess) {
-    cudaEventDestroy(ev0);
-    return fail(CRTB200_ERR_CUDA, "cudaEventCreate failed");
-  }
-  struct Events {
-    cudaEvent_t a, b;
-    ~Events() {
-      cudaEventDestroy(a);
-      cudaEventDestroy(b);
-    }
-  } events{ev0, ev1};
+  Event ev0, ev1;
+  CUDA_TRY(ev0.create(cudaEventDefault));
+  CUDA_TRY(ev1.create(cudaEventDefault));
 
   if (!r.geom.empty()) CUDA_TRY(cudaMemcpyAsync(geom, r.geom.data(), r.geom.size() * sizeof(float4), cudaMemcpyHostToDevice, st));
   CUDA_TRY(cudaMemcpyAsync(d_item_base, item_base.data(), item_base.size() * 4, cudaMemcpyHostToDevice, st));
@@ -1366,12 +1349,12 @@ static int plan_queues(crtb200_ctx *c, uint32_t shard_items, uint32_t max_depth,
   c->n_chunks = (uint32_t)((shard_items + items - 1) / items);
   if (c->cap_items == items && c->cap_depth == max_depth && c->cap_sets == n_sets && c->cap_branch == node_branching(c)) return CRTB200_OK;
   if (c->sets.size() < n_sets) c->sets.resize(n_sets);
-  if (!c->fork_ev) CUDA_TRY(cudaEventCreateWithFlags(&c->fork_ev, cudaEventDisableTiming));
+  CUDA_TRY(c->fork_ev.create(cudaEventDisableTiming));
   for (uint32_t k = 0; k < n_sets; k++) {
     crtb200_ctx::QueueSet &q = c->sets[k];
-    if (!q.stream) CUDA_TRY(cudaStreamCreateWithFlags(&q.stream, cudaStreamNonBlocking));
+    CUDA_TRY(q.stream.create(cudaStreamNonBlocking));
     apply_l2_window(c, q.stream);
-    if (!q.done) CUDA_TRY(cudaEventCreateWithFlags(&q.done, cudaEventDisableTiming));
+    CUDA_TRY(q.done.create(cudaEventDisableTiming));
     uint64_t total = 0;
     for (uint32_t l = 0; l <= max_depth; l++) {
       q.lv.offset[l] = (uint32_t)total;
@@ -1392,13 +1375,11 @@ static int plan_queues(crtb200_ctx *c, uint32_t shard_items, uint32_t max_depth,
     CUDA_TRY(q.ovf.ensure(3 * ovf_cap));
     // every record starts out "not published" (r0.x = CRT_INVALID); k_coop leaves a taken record in that state again
     CUDA_TRY(cudaMemsetAsync(q.ovf.p, 0xFF, 3 * ovf_cap * sizeof(uint4), q.stream));
-    if (!q.coop_stream) {
-      int lo = 0, hi = 0;
-      CUDA_TRY(cudaDeviceGetStreamPriorityRange(&lo, &hi));  // lo = least priority: the traversal kernel's blocks go first
-      CUDA_TRY(cudaStreamCreateWithPriority(&q.coop_stream, cudaStreamNonBlocking, lo));
-      CUDA_TRY(cudaEventCreateWithFlags(&q.coop_fork, cudaEventDisableTiming));
-      CUDA_TRY(cudaEventCreateWithFlags(&q.coop_join, cudaEventDisableTiming));
-    }
+    int lo = 0, hi = 0;
+    CUDA_TRY(cudaDeviceGetStreamPriorityRange(&lo, &hi));  // lo = least priority: the traversal kernel's blocks go first
+    CUDA_TRY(q.coop_stream.create(cudaStreamNonBlocking, lo));
+    CUDA_TRY(q.coop_fork.create(cudaEventDisableTiming));
+    CUDA_TRY(q.coop_join.create(cudaEventDisableTiming));
     // counts | work cursors | hand-off counters; every cursor / counter group on a 128-byte line of its own
     const size_t n_counts = 64, n_work = CRT_CTL_STRIDE * (CRT_MAX_LEVELS + 2), n_ovf = CRT_CTL_STRIDE * (CRT_MAX_LEVELS + 1);
     CUDA_TRY(q.ctl.ensure(n_counts + n_work + n_ovf));
@@ -1463,13 +1444,12 @@ static int plan_mask(crtb200_ctx *c, const crtb200_options *o) {
   return CRTB200_OK;
 }
 
-static cudaEvent_t next_event(crtb200_ctx *c) {
-  if (c->kev_used == c->kev.size()) {
-    cudaEvent_t e;
-    cudaEventCreate(&e);
-    c->kev.push_back(e);
-  }
-  return c->kev[c->kev_used++];
+// records the frame's next per-launch timing event on st, creating it on first use
+static cudaError_t record_next_event(crtb200_ctx *c, cudaStream_t st) {
+  if (c->kev_used == c->kev.size()) c->kev.emplace_back();
+  Event &e = c->kev[c->kev_used++];
+  const cudaError_t err = e.create(cudaEventDefault);
+  return err != cudaSuccess ? err : cudaEventRecord(e, st);
 }
 
 // dynamic shared memory of the kernels that walk one ray per lane: the visited-mesh bitset of scenes with > 64 meshes
@@ -1556,8 +1536,8 @@ static void launch_coop(crtb200_ctx *c, const Flavour &fl, const Frame &fr, crtb
     }); }); }); });
 }
 
-// One traversal launch -- k_closest of level `level`, the shadow pass, or a query kernel -- and with hand-off k_coop
-// around it (DESIGN.md 3.8).  launch(stream, coop_blocks, early) enqueues the walk source's traversal kernel
+// One traversal launch on st -- k_closest of level `level`, the shadow pass, or a query kernel -- and with hand-off
+// k_coop around it (DESIGN.md 3.8).  launch(stream, coop_blocks, early) enqueues the walk source's traversal kernel
 // (coop_blocks = 0) or its k_coop pass.  With an early pass (`early_ok`: one queue set, and not a secondary level of a
 // frame) the side stream is forked BEFORE the traversal kernel is launched; behind it k_mark marks the traversal kernel's
 // end, the early pass starts on the side stream (its blocks get SM resources as the traversal kernel's blocks exit)
@@ -1565,40 +1545,40 @@ static void launch_coop(crtb200_ctx *c, const Flavour &fl, const Frame &fr, crtb
 // per_kernel: time them (closest_ms, shadow_ms, coop_*_ms); a mark with a kind (0 closest, 1 shadow, 2 / 3 their k_coop
 // part) opens a span and the next mark closes it, collect_stats_one reads them in pairs.
 template <typename Launch>
-static int traverse(crtb200_ctx *c, bool handoff, bool early_ok, crtb200_ctx::QueueSet &q, bool shadow, uint32_t level,
-                    bool per_kernel, uint32_t &launches, const Launch &launch) {
+static int traverse(crtb200_ctx *c, bool handoff, bool early_ok, crtb200_ctx::QueueSet &q, cudaStream_t st, bool shadow,
+                    uint32_t level, bool per_kernel, uint32_t &launches, const Launch &launch) {
   auto mark = [&](int kind) {
-    if (per_kernel) cudaEventRecord(next_event(c), q.stream);
     if (per_kernel && kind >= 0) c->kev_kind.push_back(kind);
+    return per_kernel ? record_next_event(c, st) : cudaSuccess;
   };
   const bool early = handoff && c->coop_early > 0 && early_ok;
-  mark(shadow ? 1 : 0);
+  CUDA_TRY(mark(shadow ? 1 : 0));
   if (early) {
-    CUDA_TRY(cudaEventRecord(q.coop_fork, q.stream));
+    CUDA_TRY(cudaEventRecord(q.coop_fork, st));
     CUDA_TRY(cudaStreamWaitEvent(q.coop_stream, q.coop_fork, 0));
   }
-  launch(q.stream, 0, 0u);
+  launch(st, 0, 0u);
   if (handoff) {
-    mark(-1);
-    mark(shadow ? 3 : 2);
+    CUDA_TRY(mark(-1));
+    CUDA_TRY(mark(shadow ? 3 : 2));
     if (early) {
-      k_mark<<<1, 32, 0, q.stream>>>(q.lv.ovf_ctl + CRT_CTL_STRIDE * (shadow ? (uint32_t)CRT_MAX_LEVELS : level) + 24u);
+      k_mark<<<1, 32, 0, st>>>(q.lv.ovf_ctl + CRT_CTL_STRIDE * (shadow ? (uint32_t)CRT_MAX_LEVELS : level) + 24u);
       launch(q.coop_stream, c->sm_count * c->coop_early, 1u);
       CUDA_TRY(cudaEventRecord(q.coop_join, q.coop_stream));
-      CUDA_TRY(cudaStreamWaitEvent(q.stream, q.coop_join, 0));
+      CUDA_TRY(cudaStreamWaitEvent(st, q.coop_join, 0));
       launches += 2;
     }
-    launch(q.stream, c->blocks_coop, 0u);
+    launch(st, c->blocks_coop, 0u);
     launches++;
   }
-  mark(-1);
+  CUDA_TRY(mark(-1));
   return CRTB200_OK;
 }
 
 // traverse for k_closest of level `level` or the shadow pass of a frame's chunk
 static int traverse_frame(crtb200_ctx *c, const Flavour &fl, const Frame &fr, crtb200_ctx::QueueSet &q, bool shadow, uint32_t level,
                           bool per_kernel, uint32_t &launches) {
-  return traverse(c, fl.handoff, c->cap_sets == 1 && (shadow || level == 0), q, shadow, level, per_kernel, launches,
+  return traverse(c, fl.handoff, c->cap_sets == 1 && (shadow || level == 0), q, q.stream, shadow, level, per_kernel, launches,
                   [&](cudaStream_t st, int coop_blocks, uint32_t early) {
                     if (coop_blocks)
                       launch_coop(c, fl, fr, q, shadow, level, coop_blocks, st, early);
@@ -1615,7 +1595,6 @@ static int traverse_frame(crtb200_ctx *c, const Flavour &fl, const Frame &fr, cr
 static int enqueue_query(crtb200_ctx *x, const Flavour &fl, uint32_t ray_type, const QueryBatch &qb, cudaStream_t st,
                          uint32_t &launches) {
   crtb200_ctx::QueueSet &q = x->query;
-  q.stream = st;
   q.lv.tail_iters = fl.handoff ? (uint32_t)(x->tail_iters + 1) : 0u;
   q.lv.tail_start = (uint32_t)x->tail_start;
   q.lv.tail_start_closest = (uint32_t)x->tail_start_closest;
@@ -1625,7 +1604,7 @@ static int enqueue_query(crtb200_ctx *x, const Flavour &fl, uint32_t ray_type, c
   const bool shadow = ray_type == CRTB200_RAY_SHADOW, primary = ray_type == CRTB200_RAY_PRIMARY;
   uint32_t *const work = q.work + CRT_CTL_STRIDE * (shadow ? (uint32_t)CRT_MAX_LEVELS : 0u);
   launches++;
-  return traverse(x, fl.handoff, true, q, shadow, 0, false, launches, [&](cudaStream_t s, int coop_blocks, uint32_t early) {
+  return traverse(x, fl.handoff, true, q, st, shadow, 0, false, launches, [&](cudaStream_t s, int coop_blocks, uint32_t early) {
     if (coop_blocks) {
       as_const(shadow, [&](auto sh) { as_const(primary, [&](auto prim) {
         if constexpr (!(sh && prim)) k_coop_query<sh, prim><<<coop_blocks, 32 * CRT_COOP_WARPS, 0, s>>>(x->sc, q.lv, qb, early);
@@ -1669,11 +1648,10 @@ static int query_scratch(crtb200_ctx *x) {
   int lo = 0, hi = 0;
   CUDA_TRY(cudaDeviceGetStreamPriorityRange(&lo, &hi));
   // (each part is created once: a call that failed half-way is completed by the next one)
-  if (!q.coop_stream) CUDA_TRY(cudaStreamCreateWithPriority(&q.coop_stream, cudaStreamNonBlocking, lo));
-  if (!q.coop_fork) CUDA_TRY(cudaEventCreateWithFlags(&q.coop_fork, cudaEventDisableTiming));
-  if (!q.coop_join) CUDA_TRY(cudaEventCreateWithFlags(&q.coop_join, cudaEventDisableTiming));
-  for (auto &e : x->query_ev)
-    if (!e) CUDA_TRY(cudaEventCreate(&e));
+  CUDA_TRY(q.coop_stream.create(cudaStreamNonBlocking, lo));
+  CUDA_TRY(q.coop_fork.create(cudaEventDisableTiming));
+  CUDA_TRY(q.coop_join.create(cudaEventDisableTiming));
+  for (Event &e : x->query_ev) CUDA_TRY(e.create(cudaEventDefault));
   q.work = q.ctl.p;
   q.lv.ovf = q.ovf.p;
   q.lv.ovf_ctl = q.ctl.p + n_work;
@@ -1796,11 +1774,9 @@ static int copy_band(crtb200_ctx *c, const FrameReq &r, cudaStream_t qs, uint32_
   if (h.rgb8) CUDA_TRY(cudaMemcpyAsync(h.rgb8 + off * 3, r.d_rgb8 + off * 3, cnt * 3, cudaMemcpyDeviceToHost, cs));
   if (h.hits) CUDA_TRY(cudaMemcpyAsync(h.hits + off, r.d_hits + off, cnt * sizeof(HitRec), cudaMemcpyDeviceToHost, cs));
   if (getenv("CRT_CHUNK_TIMES")) {
-    while (c->dbg_ev.size() < 2 * (size_t)(chunk + 1)) {
-      cudaEvent_t e = nullptr;
-      CUDA_TRY(cudaEventCreate(&e));
-      c->dbg_ev.push_back(e);
-    }
+    if (c->dbg_ev.size() < 2 * (size_t)(chunk + 1)) c->dbg_ev.resize(2 * (size_t)(chunk + 1));
+    CUDA_TRY(c->dbg_ev[2 * chunk].create(cudaEventDefault));
+    CUDA_TRY(c->dbg_ev[2 * chunk + 1].create(cudaEventDefault));
     CUDA_TRY(cudaEventRecord(c->dbg_ev[2 * chunk], qs));
     CUDA_TRY(cudaEventRecord(c->dbg_ev[2 * chunk + 1], cs));
     c->dbg_chunks = chunk + 1;
@@ -1870,13 +1846,10 @@ static int enqueue_frame(crtb200_ctx *c, const FrameReq &r, cudaStream_t st) {
   // band copies leave on their own stream, so a set starts its next chunk while its last band is still in flight
   const bool band_stream = band_copies && n_sets > 1 && !getenv("CRT_NO_BAND_STREAM");
   if (band_stream) {
-    if (!c->band_stream) CUDA_TRY(cudaStreamCreateWithFlags(&c->band_stream, cudaStreamNonBlocking));
-    if (!c->band_done) CUDA_TRY(cudaEventCreateWithFlags(&c->band_done, cudaEventDisableTiming));
-    while (c->chunk_done.size() < c->n_chunks) {
-      cudaEvent_t e = nullptr;
-      CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-      c->chunk_done.push_back(e);
-    }
+    CUDA_TRY(c->band_stream.create(cudaStreamNonBlocking));
+    CUDA_TRY(c->band_done.create(cudaEventDisableTiming));
+    if (c->chunk_done.size() < c->n_chunks) c->chunk_done.resize(c->n_chunks);
+    for (Event &e : c->chunk_done) CUDA_TRY(e.create(cudaEventDisableTiming));
   }
   for (uint32_t begin = 0; begin < shard_items; begin += c->cap_items, chunk++) {
     crtb200_ctx::QueueSet &q = c->sets[chunk % n_sets];
@@ -2176,10 +2149,10 @@ int crtb200_render_frames(crtb200_ctx *c, const crtb200_camera *cams, uint32_t n
   }
   CUDA_TRY(c->frame_b.ensure(px * 3));
   if (rgb8_out) CUDA_TRY(c->frame8_b.ensure(px * 3));
-  if (!c->copy_stream) CUDA_TRY(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
+  CUDA_TRY(c->copy_stream.create(cudaStreamNonBlocking));
   for (int k = 0; k < 2; k++) {
-    if (!c->rendered[k]) CUDA_TRY(cudaEventCreateWithFlags(&c->rendered[k], cudaEventDisableTiming));
-    if (!c->copied[k]) CUDA_TRY(cudaEventCreateWithFlags(&c->copied[k], cudaEventDisableTiming));
+    CUDA_TRY(c->rendered[k].create(cudaEventDisableTiming));
+    CUDA_TRY(c->copied[k].create(cudaEventDisableTiming));
   }
   c->last = crtb200_stats{};
   uint32_t launches = 0;
@@ -2269,14 +2242,6 @@ struct AccumStaging {
   DevBuf<HitRec> hit;
   DevBuf<uint32_t> bad, counts;
   DevBuf<unsigned long long> tot;
-  ~AccumStaging() {
-    sum.release();
-    sumsq.release();
-    hit.release();
-    bad.release();
-    counts.release();
-    tot.release();
-  }
 };
 
 // k_accum_load on every GPU from the staged arrays (all empty: an adaptive begin's flags), then the totals the session
@@ -2642,12 +2607,11 @@ int crtb200_generate_rays(crtb200_ctx *c, const crtb200_camera *cam, float *rays
   if (n == 0) return CRTB200_OK;
   DevBuf<float> d;
   CUDA_TRY(d.ensure(n * 6));
-  int rc = crtb200_generate_rays_device(c, cam, d.p, c->stream);
-  cudaError_t e = rc ? cudaSuccess : cudaMemcpyAsync(rays_out, d.p, n * 6 * sizeof(float), cudaMemcpyDeviceToHost, c->stream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-  d.release();
-  CUDA_TRY(e);
-  return rc;
+  const int rc = crtb200_generate_rays_device(c, cam, d.p, c->stream);
+  if (rc) return rc;
+  CUDA_TRY(cudaMemcpyAsync(rays_out, d.p, n * 6 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  return CRTB200_OK;
 }
 
 int crtb200_scene_trees(crtb200_ctx *c, crtb200_trees *t) {
@@ -2714,18 +2678,13 @@ int crtb200_debug_powf5(crtb200_ctx *c, const float *x, uint32_t n, float *out) 
   if (n == 0) return CRTB200_OK;
   CUDA_TRY(cudaSetDevice(c->device));
   DevBuf<float> dx, dy;
-  cudaError_t e = dx.ensure(n);
-  if (e == cudaSuccess) e = dy.ensure(n);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(dx.p, x, (size_t)n * 4, cudaMemcpyHostToDevice, c->stream);
-  if (e == cudaSuccess) {
-    k_powf5<<<c->sm_count * 8, 256, 0, c->stream>>>(dx.p, n, dy.p);
-    e = cudaGetLastError();
-  }
-  if (e == cudaSuccess) e = cudaMemcpyAsync(out, dy.p, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-  dx.release();
-  dy.release();
-  CUDA_TRY(e);
+  CUDA_TRY(dx.ensure(n));
+  CUDA_TRY(dy.ensure(n));
+  CUDA_TRY(cudaMemcpyAsync(dx.p, x, (size_t)n * 4, cudaMemcpyHostToDevice, c->stream));
+  k_powf5<<<c->sm_count * 8, 256, 0, c->stream>>>(dx.p, n, dy.p);
+  CUDA_TRY(cudaGetLastError());
+  CUDA_TRY(cudaMemcpyAsync(out, dy.p, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
+  CUDA_TRY(cudaStreamSynchronize(c->stream));
   return CRTB200_OK;
 }
 
@@ -2838,35 +2797,26 @@ int crtb200_trace_rays(crtb200_ctx *c, const float *rays, uint32_t n, uint32_t r
   DevBuf<float> d_rays, d_dist;
   DevBuf<crtb200_hit> d_hits;
   DevBuf<uint8_t> d_occ;
-  cudaError_t e = d_rays.ensure((size_t)n * 6);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(d_rays.p, rays, (size_t)n * 6 * sizeof(float), cudaMemcpyHostToDevice, c->stream);
+  CUDA_TRY(d_rays.ensure((size_t)n * 6));
+  CUDA_TRY(cudaMemcpyAsync(d_rays.p, rays, (size_t)n * 6 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
   if (shadow) {
-    if (e == cudaSuccess) e = d_dist.ensure(n);
-    if (e == cudaSuccess) e = d_occ.ensure(n);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_dist.p, max_distance, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, c->stream);
-  } else if (e == cudaSuccess) {
-    e = d_hits.ensure(n);
+    CUDA_TRY(d_dist.ensure(n));
+    CUDA_TRY(d_occ.ensure(n));
+    CUDA_TRY(cudaMemcpyAsync(d_dist.p, max_distance, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+  } else {
+    CUDA_TRY(d_hits.ensure(n));
   }
-  if (e == cudaSuccess) {
-    b.rays = d_rays.p;
-    b.max_distance = d_dist.p;
-    b.hits = d_hits.p;
-    b.occluded = d_occ.p;
-    rc = crtb200_trace_rays_device(c, &b, c->stream);
-  }
-  if (e == cudaSuccess && rc == CRTB200_OK) {
-    if (shadow)
-      e = cudaMemcpyAsync(occluded_out, d_occ.p, n, cudaMemcpyDeviceToHost, c->stream);
-    else
-      e = cudaMemcpyAsync(hits_out, d_hits.p, (size_t)n * sizeof(crtb200_hit), cudaMemcpyDeviceToHost, c->stream);
-  }
-  if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-  d_rays.release();
-  d_dist.release();
-  d_hits.release();
-  d_occ.release();
-  CUDA_TRY(e);
-  return rc;
+  b.rays = d_rays.p;
+  b.max_distance = d_dist.p;
+  b.hits = d_hits.p;
+  b.occluded = d_occ.p;
+  if ((rc = crtb200_trace_rays_device(c, &b, c->stream))) return rc;
+  if (shadow)
+    CUDA_TRY(cudaMemcpyAsync(occluded_out, d_occ.p, n, cudaMemcpyDeviceToHost, c->stream));
+  else
+    CUDA_TRY(cudaMemcpyAsync(hits_out, d_hits.p, (size_t)n * sizeof(crtb200_hit), cudaMemcpyDeviceToHost, c->stream));
+  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  return CRTB200_OK;
 }
 
 }  // extern "C"
