@@ -364,9 +364,13 @@ CRT_DI float cull_margin_for(const Ray &r, const float mesh_mu) {
 //   behind : some far plane lies more than mu behind the origin        tf_i < -m_i         (only when `allow_behind`)
 //   beyond : some near plane lies more than mu beyond the limit        tn_i - m_i > limit
 // Both are "box inflated by mu misses the ray segment [0, limit]" written per axis; NaN / +inf operands never cull.
-template <bool CULL>
-CRT_DI bool node_test(const float4 lo, const float4 hi, const Ray &r, const float mu, const float limit, const bool allow_behind) {
-  if (r.flags & CRT_RAY_SLOW_MASK) {
+// `m` = cull_margins(r, mu), the m_i above.
+// SLOW = false: the caller knows that r is a fast ray (no CRT_RAY_SLOW_MASK flag), and the test carries neither the flag
+// test nor the select-exact path.
+CRT_DI V3 cull_margins(const Ray &r, const float mu) { return mk(mu * fabsf(r.inv.x), mu * fabsf(r.inv.y), mu * fabsf(r.inv.z)); }
+template <bool CULL, bool SLOW = true>
+CRT_DI bool node_test(const float4 lo, const float4 hi, const Ray &r, const V3 m, const float limit, const bool allow_behind) {
+  if (SLOW && (r.flags & CRT_RAY_SLOW_MASK)) {
     float t0, t1;
     return slab_test_exact(lo, hi, r, t0, t1);
   }
@@ -380,9 +384,8 @@ CRT_DI bool node_test(const float4 lo, const float4 hi, const Ray &r, const floa
   const float t1 = fminf(fminf(fminf(CRT_FLT_MAX, fx), fy), fz);
   bool pass = !(t0 > t1);
   if (CULL) {
-    const float mx = mu * fabsf(r.inv.x), my = mu * fabsf(r.inv.y), mz = mu * fabsf(r.inv.z);
-    const bool behind = allow_behind && ((fx < -mx) || (fy < -my) || (fz < -mz));
-    const bool beyond = (nx - mx > limit) || (ny - my > limit) || (nz - mz > limit);
+    const bool behind = allow_behind && ((fx < -m.x) || (fy < -m.y) || (fz < -m.z));
+    const bool beyond = fmaxf(fmaxf(nx - m.x, ny - m.y), nz - m.z) > limit;  // fmaxf drops a NaN operand, as || drops its false test
     pass = pass && !behind && !beyond;
   }
   return pass;
@@ -408,8 +411,8 @@ CRT_DI int trav_slow(Trav &s, const DScene &sc, const Ray &r);
 //   trav_slow   the bookkeeping between trees for a lane with cur == cend and no pending triangles: next mesh of the
 //               current top-level leaf, or back to the top-level tree, or TRAV_DONE.
 // Together they perform exactly the state transitions of the reference's walk.
-template <bool COUNT, bool CULL>
-CRT_DI bool trav_fast(Trav &s, const DScene &sc, const Ray &r, uint32_t &node_tests, const float limit, const bool allow_behind) {
+template <bool COUNT, bool CULL, bool SLOW>
+CRT_DI bool trav_fast(Trav &s, const DScene &sc, const Ray &r, uint32_t &node_tests, const V3 m, const float limit, const bool allow_behind) {
   const uint32_t idx = s.cur;
   const float4 lo = ld_node(&sc.nodes[2 * (size_t)idx]);
   const float4 hi = ld_node(&sc.nodes[2 * (size_t)idx + 1]);
@@ -420,7 +423,7 @@ CRT_DI bool trav_fast(Trav &s, const DScene &sc, const Ray &r, uint32_t &node_te
   if (!leaf) asm volatile("prefetch.global.L1 [%0];" ::"l"(&sc.nodes[2 * (size_t)a]));
 #endif
   if (COUNT) node_tests++;
-  const bool pass = node_test<CULL>(lo, hi, r, s.mu, limit, allow_behind);
+  const bool pass = node_test<CULL, SLOW>(lo, hi, r, m, limit, allow_behind);
   s.cur = (pass || leaf) ? idx + 1 : a;
   if (pass && leaf) {
     const uint32_t first = __float_as_uint(hi.w), last = first + (a & ~CRT_LEAF_FLAG);
@@ -445,27 +448,27 @@ CRT_DI bool trav_fast(Trav &s, const DScene &sc, const Ray &r, uint32_t &node_te
 // of a loop whose iteration time is the latency of the slowest lane's load.  When node idx fails (an inner node) the
 // second test is simply discarded; testing a node the reference would not have reached cannot change the walk,
 // because only the pass / fail of nodes that ARE reached is acted on.
-template <bool COUNT, bool CULL>
-CRT_DI bool trav_fast2(Trav &s, const DScene &sc, const Ray &r, uint32_t &node_tests, const float limit, const bool allow_behind) {
+template <bool COUNT, bool CULL, bool SLOW>
+CRT_DI bool trav_fast2(Trav &s, const DScene &sc, const Ray &r, uint32_t &node_tests, const V3 m, const float limit, const bool allow_behind) {
   const uint32_t idx = s.cur;
   const bool has2 = idx + 1u < s.cend;
   const uint32_t jdx = has2 ? idx + 1u : idx;
   const float4 lo0 = ld_node(&sc.nodes[2 * (size_t)idx]), hi0 = ld_node(&sc.nodes[2 * (size_t)idx + 1]);
   const float4 lo1 = ld_node(&sc.nodes[2 * (size_t)jdx]), hi1 = ld_node(&sc.nodes[2 * (size_t)jdx + 1]);
-  const bool pass0 = node_test<CULL>(lo0, hi0, r, s.mu, limit, allow_behind);
-  const bool pass1 = node_test<CULL>(lo1, hi1, r, s.mu, limit, allow_behind);
+  const bool pass0 = node_test<CULL, SLOW>(lo0, hi0, r, m, limit, allow_behind);
+  const bool pass1 = node_test<CULL, SLOW>(lo1, hi1, r, m, limit, allow_behind);
   const uint32_t a0 = __float_as_uint(lo0.w), a1 = __float_as_uint(lo1.w);
-  const bool leaf0 = (a0 & CRT_LEAF_FLAG) != 0u, leaf1 = (a1 & CRT_LEAF_FLAG) != 0u;
   if (COUNT) node_tests++;
   // which of the two nodes decides where the walk goes: the second one iff the first is stepped over (inner + pass, or a
-  // failing leaf) and a second one exists
-  const bool second = has2 && (pass0 != leaf0);
+  // failing leaf) and a second one exists.  The leaf flag is the sign bit of a.
+  const bool second = has2 && (pass0 != ((int32_t)a0 < 0));
   if (COUNT && second) node_tests++;
-  const uint32_t a = second ? a1 : a0, b = __float_as_uint(second ? hi1.w : hi0.w), at = second ? idx + 1u : idx;
-  const bool pass = second ? pass1 : pass0, leaf = second ? leaf1 : leaf0;
+  const uint32_t a = second ? a1 : a0, at = second ? jdx : idx;
+  // (pass as predicate logic: a ?: between two bools compiles to integer selects and a compare)
+  const bool pass = (second && pass1) || (!second && pass0), leaf = (int32_t)a < 0;
   s.cur = (pass || leaf) ? at + 1u : a;
   if (pass && leaf) {
-    const uint32_t first = b, last = first + (a & ~CRT_LEAF_FLAG);
+    const uint32_t first = __float_as_uint(second ? hi1.w : hi0.w), last = first + (a & ~CRT_LEAF_FLAG);
     if (s.below) {
       s.tref = first;
       s.tend = last;

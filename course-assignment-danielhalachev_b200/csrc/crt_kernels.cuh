@@ -23,6 +23,7 @@
 #include "crt_device.cuh"
 #include "crt_powf5.h"
 #include "crt_sampling.h"
+#include <type_traits>
 
 namespace crtd {
 
@@ -484,17 +485,29 @@ CRT_DI void walk_loop(const DScene &sc, const Frame &fr, const Levels &lv, uint3
     // ---- node phase: one AABB step per iteration while enough lanes want one ----
     bool need = active && tv.tref == tv.tend;
     const uint32_t thr = node_threshold(__popc(__ballot_sync(CRT_FULL_MASK, active)));
-    while ((uint32_t)__popc(__ballot_sync(CRT_FULL_MASK, need)) >= thr) {
-      CRT_PC_COUNT(5, 1)
+    // A lane's ray stays fixed through the phase (refill runs before it): when no stepping lane holds a ray of the
+    // select-exact slab path (CRT_RAY_SLOW_MASK: axis-parallel or non-finite components, rare), the loop runs the box
+    // test without that path, its flag test and its reconvergence point.
+    const auto node_loop = [&](auto slow) {
+      constexpr bool SLOW = decltype(slow)::value;
+      uint32_t step = need;  // a 32-bit flag: a bool carried through the loop is repacked as a byte every iteration
+      while ((uint32_t)__popc(__ballot_sync(CRT_FULL_MASK, step)) >= thr) {
+        CRT_PC_COUNT(5, 1)
 #if CRT_PHASE_CLOCKS
-      if (need) ray_iters++;
+        if (step) ray_iters++;
 #endif
-      if (need) {
-        walk_iters++;
-        need = CRT_NODE_PAIR ? trav_fast2<COUNT, CULL>(tv, sc, ray, n_nodes, w.limit(), w.allow_behind())
-                             : trav_fast<COUNT, CULL>(tv, sc, ray, n_nodes, w.limit(), w.allow_behind());
+        if (step) {
+          walk_iters++;
+          step = CRT_NODE_PAIR ? trav_fast2<COUNT, CULL, SLOW>(tv, sc, ray, n_nodes, cull_margins(ray, tv.mu), w.limit(), w.allow_behind())
+                               : trav_fast<COUNT, CULL, SLOW>(tv, sc, ray, n_nodes, cull_margins(ray, tv.mu), w.limit(), w.allow_behind());
+        }
       }
-    }
+      need = step;
+    };
+    if (__any_sync(CRT_FULL_MASK, need && (ray.flags & CRT_RAY_SLOW_MASK)))
+      node_loop(std::true_type());
+    else
+      node_loop(std::false_type());
     CRT_PC_MARK(2)
     // ---- triangle phase: all pending leaves, packed across the warp ----
     const bool parked = active && tv.tref != tv.tend;
@@ -1171,7 +1184,7 @@ CRT_DI void coop_walks(const DScene &sc, const Levels &lv, const uint32_t level,
           const float4 lo = ld_node(&sc.nodes[2 * (size_t)cur]), hi = ld_node(&sc.nodes[2 * (size_t)cur + 1]);
           const uint32_t a = __float_as_uint(lo.w);
           const bool leaf = (a & CRT_LEAF_FLAG) != 0u;
-          const bool pass = node_test<false>(lo, hi, ray, CRT_INF, CRT_INF, false);
+          const bool pass = node_test<false>(lo, hi, ray, mk(CRT_INF, CRT_INF, CRT_INF), CRT_INF, false);
           cur = (pass || leaf) ? cur + 1u : a;
           if (pass && leaf) {
             mref = __float_as_uint(hi.w);
@@ -1232,7 +1245,7 @@ CRT_DI void coop_walks(const DScene &sc, const Levels &lv, const uint32_t level,
         b = __float_as_uint(hi.w);
         const bool leaf = (a & CRT_LEAF_FLAG) != 0u;
         const uint32_t endj = leaf ? j + 1u : a;
-        if (endj > from && node_test<CULL>(lo, hi, ray, mu, lim, SHADOW || lim < CRT_INF)) {
+        if (endj > from && node_test<CULL>(lo, hi, ray, cull_margins(ray, mu), lim, SHADOW || lim < CRT_INF)) {
           leaf_hit = leaf;
           if (!leaf) cnt = (b != CRT_INVALID) ? 2u : 1u;
         }
