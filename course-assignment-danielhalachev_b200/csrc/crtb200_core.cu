@@ -56,8 +56,8 @@ struct ErrScope {
   ~ErrScope() { g_error_ctx = prev; }
 };
 
-// One helper thread per peer GPU of a multi-GPU context: launches are asynchronous, but issuing a frame's ~20 launches
-// takes the host ~0.1 ms per GPU, which eight GPUs cannot afford serially when a shard renders in ~0.5 ms.
+// One helper thread per GPU after the first of a multi-GPU context: launches are asynchronous, but issuing a frame's
+// ~20 launches takes the host ~0.1 ms per GPU, which eight GPUs cannot afford serially when a shard renders in ~0.5 ms.
 struct Worker {
   std::thread th;
   std::mutex m;
@@ -173,16 +173,42 @@ using Event = CudaHandle<cudaEvent_t>;
 // counters of a render kept beside crtb200_stats: diffuse rays, and an adaptive step's pixel-samples and stopped pixels
 struct SideCounts { uint64_t diffuse = 0, px_samples = 0, stopped = 0; };
 
-struct crtb200_ctx {
+// What a render or query counted: crtb200_stats and the side counts.  Read from one GPU's CRT_STAT_* slots it holds
+// the counters only; totals add launches and times too.
+struct Counts {
+  crtb200_stats s{};
+  SideCounts side;
+};
+
+// queues: `concurrency` independent buffer sets, each with its own stream.  Consecutive chunks of a frame go to the
+// sets round-robin, so the latency-bound tails of one chunk's persistent kernels (and the small secondary-level
+// launches of reflective / refractive scenes) are filled by the other chunks' kernels.
+struct QueueSet {
+  Levels lv{};
+  DevBuf<float4> ray_o, ray_d, color, dq;
+  DevBuf<uint32_t> hit_tri, ctl;  // ctl = counts | work cursors | hand-off counters, zeroed by one memset per chunk
+  DevBuf<float> hit_t;
+  DevBuf<uint4> comb;
+  DevBuf<uint8_t> vis;
+  DevBuf<uint4> ovf;          // walks handed off to k_coop (3 x uint4 per record)
+  DevBuf<float4> acc;         // GI frames: per level-0 item of the chunk, the running sample sum (k_sample_acc)
+  DevBuf<uint2> hit0;         //            ... and sample 0's primary hit
+  DevBuf<uint32_t> alist, acount;  // adaptive passes: the chunk's active shard items and their count (k_adapt_compact)
+  uint32_t *work = nullptr;   // into ctl
+  Stream stream;              // (frames only: a query runs on the caller's stream)
+  Event done;
+  // early k_coop pass: low-priority side stream, forked before and joined behind every traversal launch
+  Stream coop_stream;
+  Event coop_fork, coop_join;
+};
+
+// One GPU of a context: what each GPU of a multi-GPU context holds for itself -- its stream, scene replica, queues,
+// query scratch, progressive accumulator shard and tuning.
+struct Gpu {
   int device = 0;
   int sm_count = 0;
   Stream stream;
-  Event ev[2];                // the last frame's span on the caller's stream
-  std::vector<Event> kev;     // per-launch event pairs: K2 / K3 timing
-  std::vector<int> kev_kind;  // 0 = closest, 1 = shadow, 2 / 3 their k_coop part (one entry per pair)
-  size_t kev_used = 0;
   bool have_scene = false;
-  uint64_t queue_budget = 16ull << 30;
 
   // scene
   DScene sc{};
@@ -217,8 +243,61 @@ struct crtb200_ctx {
   DevBuf<float> texels;
   DevBuf<DLight> lights;
   bool has_reflective = false, has_refractive = false;
-  uint64_t scene_bytes = 0;
   uint32_t n_nodes = 0, n_leaf_refs = 0, n_top_refs = 0;  // of the uploaded scene (crtb200_debug_scene_layout)
+  uint32_t n_triangles = 0;   // of the uploaded scene (crtb200_accum_load checks the hit records it is given)
+
+  DevBuf<uint8_t> mask;
+  std::vector<crtb200_rect> mask_rects;
+  bool mask_valid = false, mask_needed = false;
+
+  // frame queues and their plan
+  std::vector<QueueSet> sets;
+  Event fork_ev;
+  DevBuf<unsigned long long> stats_dev;
+  uint32_t cap_items = 0;
+  uint32_t cap_depth = 0xFFFFFFFFu;
+  uint32_t cap_sets = 0;
+  uint32_t cap_branch = 0;    // worst-case children per ray-tree node the queues were planned for
+  uint32_t n_chunks = 0;  // chunks of the current plan (chunk k runs on set k % cap_sets)
+  uint32_t launches = 0;  // kernel launches of this GPU's part of the last frame
+  // blocks per SM of k_coop's early pass (0 = final pass only); env CRT_COOP_EARLY.  Used for the primary level and the
+  // shadow pass of frames that run on ONE stream (device frames, tile shards): with several chunk streams the tails
+  // already overlap other chunks' work and waiting blocks would only take SM resources from them (run r2ad: 4.1 -> 8 ms);
+  // the small secondary levels pay more for the extra launches and joins than they gain (hw11_room +2 %)
+  int coop_early = CRT_COOP_MIN_BLOCKS;
+  int blocks_closest = 0, blocks_closest_sec = 0, blocks_shadow = 0, blocks_coop = 0;
+
+  // caller-supplied ray batches (crtb200_trace_rays_device, DESIGN.md 3.12): the query's own scratch on this GPU, a
+  // QueueSet without ray queues or stream (work cursors and hand-off counters in ctl, hand-off records in ovf, the
+  // early k_coop pass's side stream), its device counters and grid sizes
+  QueueSet query;
+  DevBuf<unsigned long long> query_stats_dev;
+  int blocks_query_closest = 0, blocks_query_shadow = 0;
+  bool query_ready = false;  // every part of the query scratch exists (set last by query_scratch)
+
+  // progressive session: the accumulator of this GPU's tile shard, indexed by shard item
+  DevBuf<float4> acc_sum, acc_sumsq;  // S and Q
+  DevBuf<uint2> acc_hit;              // sample 0's primary hit {global triangle, bits(t)}
+
+  Event multi_done;  // (GPUs after the first) its part of a multi-GPU pass is enqueued
+};
+
+// A context: one GPU, or several (crtb200_create_multi), and what exists once for all of them.  A multi-GPU frame's
+// 8x4-pixel tiles are dealt round-robin over gpus (scene replicated); every GPU's k_store writes its pixels STRAIGHT
+// into the first GPU's frame buffers through peer-mapped pointers (NVLink / NVSwitch), so no slab, gather or assemble
+// pass exists.
+struct crtb200_ctx {
+  std::vector<std::unique_ptr<Gpu>> gpus;  // gpus[0]: the first GPU, which holds the frame and the caller's results
+  std::vector<std::unique_ptr<Worker>> workers;  // workers[i - 1] enqueues for gpus[i]
+  Event multi_fork;  // position of the caller's stream the other GPUs wait for before a multi-GPU pass
+
+  // settings
+  uint64_t queue_budget = 16ull << 30;
+  uint32_t concurrency = 2;  // chunk streams of a host-bound frame (tools/e2e_time.py, run r2aq: 2 streams with one chunk each
+                             // at 1080p, two each at 4K; 4 streams x 2 chunks cost 1080p frames 15-17 %)
+  // sampling contract (crtb200_set_sampling); sampling.use_gi = 0: unsampled frames
+  crtb200_sampling sampling{};
+
   // crtb200_upload_geometry: the trees it built, in the reference's numbering, kept on the first GPU of the context for
   // crtb200_scene_trees (40 bytes per node and 4 per mesh leaf reference; the top-level references are top_refs)
   bool trees_built = false;
@@ -227,7 +306,7 @@ struct crtb200_ctx {
   std::vector<crtb200_mesh> kd_meshes;
   crtb200_trees kd_counts{};
 
-  // frame
+  // frame, on the first GPU
   DevBuf<float> frame;   // persistent colour buffer (RayTracer::colorBuffer, RayTracer.h:69)
   DevBuf<uint8_t> frame8;
   // crtb200_render_frames: frames alternate between (frame, frame8) and (frame_b, frame8_b); the device->host copy of
@@ -237,101 +316,55 @@ struct crtb200_ctx {
   Stream copy_stream;
   Event rendered[2], copied[2];
   DevBuf<HitRec> hits;
-  DevBuf<uint8_t> mask;
-  std::vector<crtb200_rect> mask_rects;
-  bool mask_valid = false, mask_needed = false;
-
-  // queues: `concurrency` independent buffer sets, each with its own stream.  Consecutive chunks of a frame go to the
-  // sets round-robin, so the latency-bound tails of one chunk's persistent kernels (and the small secondary-level
-  // launches of reflective / refractive scenes) are filled by the other chunks' kernels.
-  struct QueueSet {
-    Levels lv{};
-    DevBuf<float4> ray_o, ray_d, color, dq;
-    DevBuf<uint32_t> hit_tri, ctl;  // ctl = counts | work cursors | hand-off counters, zeroed by one memset per chunk
-    DevBuf<float> hit_t;
-    DevBuf<uint4> comb;
-    DevBuf<uint8_t> vis;
-    DevBuf<uint4> ovf;          // walks handed off to k_coop (3 x uint4 per record)
-    DevBuf<float4> acc;         // GI frames: per level-0 item of the chunk, the running sample sum (k_sample_acc)
-    DevBuf<uint2> hit0;         //            ... and sample 0's primary hit
-    DevBuf<uint32_t> alist, acount;  // adaptive passes: the chunk's active shard items and their count (k_adapt_compact)
-    uint32_t *work = nullptr;   // into ctl
-    Stream stream;              // (frames only: a query runs on the caller's stream)
-    Event done;
-    // early k_coop pass: low-priority side stream, forked before and joined behind every traversal launch
-    Stream coop_stream;
-    Event coop_fork, coop_join;
-  };
-  std::vector<QueueSet> sets;
-  // caller-supplied ray batches (crtb200_trace_rays_device, DESIGN.md 3.12): the query's own scratch on this GPU, a
-  // QueueSet without ray queues or stream (work cursors and hand-off counters in ctl, hand-off records in ovf, the
-  // early k_coop pass's side stream), its device counters and grid sizes; on the first GPU of the context also the
-  // last query's span, GPU count and statistics
-  QueueSet query;
-  DevBuf<unsigned long long> query_stats_dev;
-  int blocks_query_closest = 0, blocks_query_shadow = 0;
-  bool query_ready = false;  // every part of the query scratch exists (set last by query_scratch)
-  Event query_ev[2];
-  uint32_t query_gpus = 0;
-  bool query_pending = false;
-  crtb200_stats query_last{};
-  uint32_t concurrency = 2;  // chunk streams of a host-bound frame (tools/e2e_time.py, run r2aq: 2 streams with one chunk each
-                             // at 1080p, two each at 4K; 4 streams x 2 chunks cost 1080p frames 15-17 %)
-  Event fork_ev;
-  DevBuf<unsigned long long> stats_dev;
-  uint32_t cap_items = 0;
-  uint32_t cap_depth = 0xFFFFFFFFu;
-  uint32_t cap_sets = 0;
-  // blocks per SM of k_coop's early pass (0 = final pass only); env CRT_COOP_EARLY.  Used for the primary level and the
-  // shadow pass of frames that run on ONE stream (device frames, tile shards): with several chunk streams the tails
-  // already overlap other chunks' work and waiting blocks would only take SM resources from them (run r2ad: 4.1 -> 8 ms);
-  // the small secondary levels pay more for the extra launches and joins than they gain (hw11_room +2 %)
-  int coop_early = CRT_COOP_MIN_BLOCKS;
-  uint32_t n_chunks = 0;  // chunks of the current plan (chunk k runs on set k % cap_sets)
   Stream band_stream;  // device -> host band copies of a chunked host-bound frame
   Event band_done;
   std::vector<Event> chunk_done;
   std::vector<Event> dbg_ev;  // CRT_CHUNK_TIMES (tools): per chunk, end of k_store and end of its band copy
   uint32_t dbg_chunks = 0;
 
-  int blocks_closest = 0, blocks_closest_sec = 0, blocks_shadow = 0, blocks_coop = 0;
+  // the last render: its span on the caller's stream, per-launch K2 / K3 timing events of the first GPU, statistics
+  Event ev[2];
+  std::vector<Event> kev;     // per-launch event pairs
+  std::vector<int> kev_kind;  // 0 = closest, 1 = shadow, 2 / 3 their k_coop part (one entry per pair)
+  size_t kev_used = 0;
   crtb200_stats last{};
-  bool last_pending = false;
-  bool bands_copied = false;  // the last enqueue_frame copied its host destinations band by band
-  // sampling contract (crtb200_set_sampling); sampling.use_gi = 0: unsampled frames
-  crtb200_sampling sampling{};
-  uint32_t frame_offset = 0;  // crtb200_render_frames: added to sampling.frame_index for frame f
   SideCounts last_side;
   uint32_t last_samples = 1;
-  uint32_t cap_branch = 0;    // worst-case children per ray-tree node the queues were planned for
-  uint32_t n_triangles = 0;   // of the uploaded scene (crtb200_accum_load checks the hit records it is given)
+  uint32_t frame_gpus = 1;     // GPUs whose device counters hold the last render's
+  bool last_pending = false;   // crtb200_render_device: statistics not collected yet
+  bool bands_copied = false;  // the last enqueue_frame copied its host destinations band by band
 
-  // progressive session (crtb200_accum_*, DESIGN.md 3.10.1): the snapshots live on the primary, and every GPU of the
-  // context keeps the accumulator of its own tile shard, indexed by shard item
+  // the last query (crtb200_trace_rays_device): span, GPU count and statistics
+  Event query_ev[2];
+  uint32_t query_gpus = 0;
+  bool query_pending = false;
+  crtb200_stats query_last{};
+
+  // progressive session (crtb200_accum_*, DESIGN.md 3.10.1): the snapshots; each GPU keeps the accumulator of its own
+  // tile shard
   bool acc_active = false;
   crtb200_camera acc_cam{};
   crtb200_options acc_opt{};
   std::vector<crtb200_rect> acc_rects;
   crtb200_sampling acc_smp{};
   uint32_t acc_done = 0;           // samples in the accumulator
-  DevBuf<float4> acc_sum, acc_sumsq;  // S and Q
-  DevBuf<uint2> acc_hit;              // sample 0's primary hit {global triangle, bits(t)}
   // adaptive session (crtb200_accum_begin_adaptive, DESIGN.md 3.10.2): the stop rule's parameters, and totals kept on
   // the host from each step's counters
   bool acc_adaptive = false;
   AdaptParams acc_ap{};
   uint64_t acc_covered = 0, acc_active_px = 0, acc_px_samples = 0;
 
-  // multi-GPU (crtb200_create_multi): this context is the primary (device_ids[0]).  A frame's 8x4-pixel tiles are dealt
-  // round-robin over primary + peers (scene replicated); every GPU's k_store writes its pixels STRAIGHT into the
-  // primary's frame buffers through peer-mapped pointers (NVLink / NVSwitch), so no slab, gather or assemble pass exists.
-  std::vector<crtb200_ctx *> peers;
-  std::vector<std::unique_ptr<Worker>> workers;
-  std::vector<int> worker_rc;
-  std::vector<std::string> worker_msg;
-  Event multi_fork;  // primary stream position the peers must wait for before touching the frame
-  Event multi_done;  // (on a peer) its shard is stored
   std::string error;                 // last error of a call on this context (crtb200_last_error_ctx)
+
+  // joins the helper threads, then frees the GPUs after the first before it: their kernels store into its memory
+  ~crtb200_ctx() {
+    workers.clear();
+    for (size_t i = gpus.size(); i-- > 0;) {
+      cudaSetDevice(gpus[i]->device);  // the members free their buffers, streams and events on this device
+      cudaStreamSynchronize(gpus[i]->stream);
+      if (i) gpus[i].reset();
+    }
+  }
 };
 static void note_ctx_error(crtb200_ctx *c, const std::string &msg) { c->error = msg; }
 
@@ -352,9 +385,11 @@ int crtb200_device_count(int *count) {
   return CRTB200_OK;
 }
 
-int crtb200_create(int device, crtb200_ctx **out) {
-  if (!out) return fail(CRTB200_ERR_ARG, "out is null");
-  *out = nullptr;
+}  // extern "C"
+
+// Adds GPU `device` to context c: device check, stream, occupancy grid sizes, tuning environment and, for a GPU after
+// the first, access to the first GPU's memory (its kernels store into the first GPU's frame).
+static int add_gpu(crtb200_ctx *c, int device) {
   int n = 0;
   CUDA_TRY(cudaGetDeviceCount(&n));
   if (device < 0 || device >= n) return fail(CRTB200_ERR_CUDA, "no such CUDA device (this library has no CPU fallback)");
@@ -363,43 +398,79 @@ int crtb200_create(int device, crtb200_ctx **out) {
   CUDA_TRY(cudaGetDeviceProperties(&prop, device));
   if (prop.major < 10)
     return fail(CRTB200_ERR_CUDA, std::string("device ") + prop.name + " is not sm_100-class; libcrtb200 is built for sm_100a only");
-  crtb200_ctx *c = new crtb200_ctx();
-  c->device = device;
-  c->sm_count = prop.multiProcessorCount;
-  if (c->stream.create(cudaStreamNonBlocking) != cudaSuccess || c->ev[0].create(cudaEventDefault) != cudaSuccess ||
-      c->ev[1].create(cudaEventDefault) != cudaSuccess) {
-    delete c;
-    return fail(CRTB200_ERR_CUDA, "cudaStreamCreate / cudaEventCreate failed");
-  }
+  c->gpus.emplace_back(new Gpu());
+  Gpu &g = *c->gpus.back();
+  g.device = device;
+  g.sm_count = prop.multiProcessorCount;
+  if (g.stream.create(cudaStreamNonBlocking) != cudaSuccess) return fail(CRTB200_ERR_CUDA, "cudaStreamCreate / cudaEventCreate failed");
   int occ = 0;
   cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_closest<true, false, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, false, false>, CRT_TRAV_BLOCK, 0);
-  c->blocks_closest = std::max(1, occ) * c->sm_count;
+  g.blocks_closest = std::max(1, occ) * g.sm_count;
   cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_closest<false, false, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, false, false>, CRT_TRAV_BLOCK, 0);
-  c->blocks_closest_sec = std::max(1, occ) * c->sm_count;
+  g.blocks_closest_sec = std::max(1, occ) * g.sm_count;
   cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_shadow<0, CRT_REFILL_SHADOW, CRT_LOOP_MODE, false, false>, CRT_TRAV_BLOCK, 0);
-  c->blocks_shadow = std::max(1, occ) * c->sm_count;
+  g.blocks_shadow = std::max(1, occ) * g.sm_count;
   cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_coop<true, false, true, CRT_COOP_GROUP>, 32 * CRT_COOP_WARPS, 0);
-  c->blocks_coop = std::max(1, occ) * c->sm_count;
+  g.blocks_coop = std::max(1, occ) * g.sm_count;
   if (const char *env = getenv("CRT_BLOCKS_PER_SM")) {  // tuning only (tools/): resident persistent CTAs per SM
     const int b = atoi(env);
-    if (b > 0) c->blocks_closest = c->blocks_closest_sec = c->blocks_shadow = b * c->sm_count;
+    if (b > 0) g.blocks_closest = g.blocks_closest_sec = g.blocks_shadow = b * g.sm_count;
   }
-  if (const char *env = getenv("CRT_L2_PERSIST")) c->l2_persist = atoi(env);
-  if (const char *env = getenv("CRT_TAIL_ITERS")) c->tail_iters = std::max(-1, atoi(env));
-  if (const char *env = getenv("CRT_TAIL_CAP")) c->tail_cap = std::max(1, atoi(env));
-  if (const char *env = getenv("CRT_TAIL_START")) c->tail_start = c->tail_start_closest = std::max(0, atoi(env));
-  if (const char *env = getenv("CRT_TAIL_START_CLOSEST")) c->tail_start_closest = std::max(0, atoi(env));
-  if (const char *env = getenv("CRT_TAIL_SMALL")) c->tail_small = std::max(0, atoi(env));
-  if (const char *env = getenv("CRT_COOP_EARLY")) c->coop_early = std::max(0, std::min(CRT_COOP_MIN_BLOCKS, atoi(env)));
-  c->l2_persist_max = (size_t)std::max(0, prop.persistingL2CacheMaxSize);
-  c->l2_window_max = (size_t)std::max(0, prop.accessPolicyMaxWindowSize);
-  if (c->l2_persist && c->l2_persist_max)
-    cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, c->l2_persist_max);  // best effort: a refusal only loses the hint
+  if (const char *env = getenv("CRT_L2_PERSIST")) g.l2_persist = atoi(env);
+  if (const char *env = getenv("CRT_TAIL_ITERS")) g.tail_iters = std::max(-1, atoi(env));
+  if (const char *env = getenv("CRT_TAIL_CAP")) g.tail_cap = std::max(1, atoi(env));
+  if (const char *env = getenv("CRT_TAIL_START")) g.tail_start = g.tail_start_closest = std::max(0, atoi(env));
+  if (const char *env = getenv("CRT_TAIL_START_CLOSEST")) g.tail_start_closest = std::max(0, atoi(env));
+  if (const char *env = getenv("CRT_TAIL_SMALL")) g.tail_small = std::max(0, atoi(env));
+  if (const char *env = getenv("CRT_COOP_EARLY")) g.coop_early = std::max(0, std::min(CRT_COOP_MIN_BLOCKS, atoi(env)));
+  g.l2_persist_max = (size_t)std::max(0, prop.persistingL2CacheMaxSize);
+  g.l2_window_max = (size_t)std::max(0, prop.accessPolicyMaxWindowSize);
+  if (g.l2_persist && g.l2_persist_max)
+    cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, g.l2_persist_max);  // best effort: a refusal only loses the hint
   if (getenv("CRT_VERBOSE"))
     fprintf(stderr, "[crtb200] %s: %d SMs, L2 %d MiB, persisting L2 max %zu MiB, access-policy window max %zu MiB, persist %s\n", prop.name,
-            prop.multiProcessorCount, prop.l2CacheSize >> 20, c->l2_persist_max >> 20, c->l2_window_max >> 20, c->l2_persist ? "on" : "off");
-  *out = c;
+            prop.multiProcessorCount, prop.l2CacheSize >> 20, g.l2_persist_max >> 20, g.l2_window_max >> 20, g.l2_persist ? "on" : "off");
+  if (c->gpus.size() == 1) return CRTB200_OK;
+  const int first = c->gpus[0]->device;
+  if (device != first) {
+    int can = 0;
+    cudaError_t e = cudaDeviceCanAccessPeer(&can, device, first);
+    if (e == cudaSuccess && !can) e = cudaErrorPeerAccessUnsupported;
+    if (e == cudaSuccess) e = cudaDeviceEnablePeerAccess(first, 0);
+    if (e == cudaErrorPeerAccessAlreadyEnabled) {
+      cudaGetLastError();
+      e = cudaSuccess;
+    }
+    if (e != cudaSuccess)
+      return fail(CRTB200_ERR_CUDA, std::string("peer access from device ") + std::to_string(device) + " to device " +
+                                        std::to_string(first) + ": " + cudaGetErrorString(e));
+  }
+  if (g.multi_done.create(cudaEventDisableTiming) != cudaSuccess) return fail(CRTB200_ERR_CUDA, "cudaEventCreate failed");
+  c->workers.emplace_back(new Worker());
   return CRTB200_OK;
+}
+
+// A context over the devices ids[0..n), the first device's current on return
+static int create(const int *ids, int n, crtb200_ctx **out) {
+  std::unique_ptr<crtb200_ctx> c(new crtb200_ctx());
+  for (int i = 0; i < n; i++) {
+    const int rc = add_gpu(c.get(), ids[i]);
+    if (rc) return rc;
+    if (i == 0 && (c->ev[0].create(cudaEventDefault) != cudaSuccess || c->ev[1].create(cudaEventDefault) != cudaSuccess))
+      return fail(CRTB200_ERR_CUDA, "cudaStreamCreate / cudaEventCreate failed");
+  }
+  cudaSetDevice(ids[0]);
+  if (n > 1 && c->multi_fork.create(cudaEventDisableTiming) != cudaSuccess) return fail(CRTB200_ERR_CUDA, "cudaEventCreate failed");
+  *out = c.release();
+  return CRTB200_OK;
+}
+
+extern "C" {
+
+int crtb200_create(int device, crtb200_ctx **out) {
+  if (!out) return fail(CRTB200_ERR_ARG, "out is null");
+  *out = nullptr;
+  return create(&device, 1, out);
 }
 
 const char *crtb200_last_error_ctx(const crtb200_ctx *c) { return c ? c->error.c_str() : g_error.c_str(); }
@@ -408,62 +479,18 @@ int crtb200_create_multi(const int *device_ids, int n, crtb200_ctx **out) {
   if (!out) return fail(CRTB200_ERR_ARG, "out is null");
   *out = nullptr;
   if (!device_ids || n < 1 || n > 64) return fail(CRTB200_ERR_ARG, "device list is null or its length is not in 1..64");
-  crtb200_ctx *c = nullptr;
-  int rc = crtb200_create(device_ids[0], &c);
-  if (rc) return rc;
-  for (int i = 1; i < n; i++) {
-    crtb200_ctx *p = nullptr;
-    rc = crtb200_create(device_ids[i], &p);
-    if (rc == CRTB200_OK && p->device != c->device) {
-      // the peer's kernels store into the primary's frame: map the primary's memory into the peer's address space
-      int can = 0;
-      cudaSetDevice(p->device);
-      cudaError_t e = cudaDeviceCanAccessPeer(&can, p->device, c->device);
-      if (e == cudaSuccess && !can) e = cudaErrorPeerAccessUnsupported;
-      if (e == cudaSuccess) e = cudaDeviceEnablePeerAccess(c->device, 0);
-      if (e == cudaErrorPeerAccessAlreadyEnabled) {
-        cudaGetLastError();
-        e = cudaSuccess;
-      }
-      if (e != cudaSuccess)
-        rc = fail(CRTB200_ERR_CUDA, std::string("peer access from device ") + std::to_string(p->device) + " to device " +
-                                        std::to_string(c->device) + ": " + cudaGetErrorString(e));
-    }
-    if (rc == CRTB200_OK && p->multi_done.create(cudaEventDisableTiming) != cudaSuccess)
-      rc = fail(CRTB200_ERR_CUDA, "cudaEventCreate failed");
-    if (rc) {
-      if (p) crtb200_destroy(p);
-      crtb200_destroy(c);
-      return rc;
-    }
-    c->peers.push_back(p);
-    c->workers.emplace_back(new Worker());
-  }
-  c->worker_rc.assign(c->peers.size(), 0);
-  c->worker_msg.assign(c->peers.size(), std::string());
-  cudaSetDevice(c->device);
-  if (!c->peers.empty() && c->multi_fork.create(cudaEventDisableTiming) != cudaSuccess) {
-    crtb200_destroy(c);
-    return fail(CRTB200_ERR_CUDA, "cudaEventCreate failed");
-  }
-  *out = c;
-  return CRTB200_OK;
+  return create(device_ids, n, out);
 }
 
 int crtb200_device_list(const crtb200_ctx *c, int *device_ids, int capacity, int *count) {
   if (!c || !count) return fail(CRTB200_ERR_ARG, "null argument");
-  *count = 1 + (int)c->peers.size();
+  *count = (int)c->gpus.size();
   if (device_ids)
-    for (int i = 0; i < capacity && i < *count; i++) device_ids[i] = i == 0 ? c->device : c->peers[i - 1]->device;
+    for (int i = 0; i < capacity && i < *count; i++) device_ids[i] = c->gpus[i]->device;
   return CRTB200_OK;
 }
 
 int crtb200_destroy(crtb200_ctx *c) {
-  if (!c) return CRTB200_OK;
-  c->workers.clear();  // joins the helper threads
-  for (crtb200_ctx *p : c->peers) crtb200_destroy(p);  // first: their kernels store into this context's memory
-  cudaSetDevice(c->device);  // the members free their buffers, streams and events on this device
-  cudaStreamSynchronize(c->stream);
   delete c;
   return CRTB200_OK;
 }
@@ -473,8 +500,7 @@ int crtb200_set_concurrency(crtb200_ctx *c, uint32_t chunks_in_flight) {
   if (!c) return fail(CRTB200_ERR_ARG, "ctx is null");
   if (chunks_in_flight < 1 || chunks_in_flight > 16) return fail(CRTB200_ERR_ARG, "concurrency must be 1..16");
   c->concurrency = chunks_in_flight;
-  c->cap_items = 0;
-  for (crtb200_ctx *p : c->peers) crtb200_set_concurrency(p, chunks_in_flight);
+  for (auto &g : c->gpus) g->cap_items = 0;
   return CRTB200_OK;
 }
 
@@ -489,7 +515,6 @@ int crtb200_set_sampling(crtb200_ctx *c, const crtb200_sampling *s) {
     v.use_gi = 1;
   }
   c->sampling = v;
-  for (crtb200_ctx *p : c->peers) crtb200_set_sampling(p, &v);
   return CRTB200_OK;
 }
 
@@ -510,8 +535,7 @@ int crtb200_set_queue_budget(crtb200_ctx *c, uint64_t bytes) {
   if (!c) return fail(CRTB200_ERR_ARG, "ctx is null");
   if (bytes < (64ull << 20)) return fail(CRTB200_ERR_ARG, "queue budget must be at least 64 MiB");
   c->queue_budget = bytes;
-  c->cap_items = 0;
-  for (crtb200_ctx *p : c->peers) crtb200_set_queue_budget(p, bytes);
+  for (auto &g : c->gpus) g->cap_items = 0;
   return CRTB200_OK;
 }
 
@@ -665,14 +689,8 @@ static float mesh_cull_margin(const crtb200_scene *s, const crtb200_mesh &me, bo
 
 }  // extern "C"
 
-static int upload_one(crtb200_ctx *c, const crtb200_scene *s);
-
-// the context and its peers, primary first: GPU i renders tile shard i
-static std::vector<crtb200_ctx *> all_gpus(crtb200_ctx *c) {
-  std::vector<crtb200_ctx *> gpus{c};
-  gpus.insert(gpus.end(), c->peers.begin(), c->peers.end());
-  return gpus;
-}
+static int upload_one(crtb200_ctx *c, Gpu &g, const crtb200_scene *s);
+static int upload_geometry_one(crtb200_ctx *c, Gpu &g, const crtb200_scene *s, bool keep);
 
 // ends the progressive session of a context and frees its accumulators on every GPU
 static void accum_release(crtb200_ctx *c) {
@@ -681,34 +699,65 @@ static void accum_release(crtb200_ctx *c) {
   c->acc_done = 0;
   c->acc_covered = c->acc_active_px = c->acc_px_samples = 0;
   c->acc_rects.clear();
-  for (crtb200_ctx *x : all_gpus(c)) {
-    cudaSetDevice(x->device);
-    x->acc_sum.release();
-    x->acc_sumsq.release();
-    x->acc_hit.release();
+  for (auto &g : c->gpus) {
+    cudaSetDevice(g->device);
+    g->acc_sum.release();
+    g->acc_sumsq.release();
+    g->acc_hit.release();
   }
-  cudaSetDevice(c->device);
+  cudaSetDevice(c->gpus[0]->device);
 }
 
-// runs fn(peer index, peer) on every peer's helper thread and fn0 on the calling thread; first error wins
-template <typename F0, typename F>
-static int on_all_devices(crtb200_ctx *c, F0 fn0, F fn) {
-  for (size_t i = 0; i < c->peers.size(); i++) {
-    c->workers[i]->post([c, i, &fn] {
-      ErrScope scope(c->peers[i]);
-      c->worker_rc[i] = fn(i, c->peers[i]);
-      c->worker_msg[i] = c->worker_rc[i] ? g_error : std::string();
+// runs fn(i, gpus[i]) for every GPU of the context, i > 0 on GPU i's helper thread and i = 0 on the calling thread;
+// first error wins, a later GPU's prefixed with its device
+template <typename F>
+static int on_all_devices(crtb200_ctx *c, F fn) {
+  const size_t n = c->gpus.size();
+  std::vector<int> rcs(n, 0);
+  std::vector<std::string> msgs(n);
+  for (size_t i = 1; i < n; i++) {
+    c->workers[i - 1]->post([&, i] {
+      rcs[i] = fn(i, *c->gpus[i]);
+      if (rcs[i]) msgs[i] = g_error;
     });
   }
-  int rc = fn0();
-  for (size_t i = 0; i < c->peers.size(); i++) {
-    c->workers[i]->wait();
-    if (rc == CRTB200_OK && c->worker_rc[i]) rc = fail(c->worker_rc[i], "device " + std::to_string(c->peers[i]->device) + ": " + c->worker_msg[i]);
+  int rc = fn(0, *c->gpus[0]);
+  for (size_t i = 1; i < n; i++) {
+    c->workers[i - 1]->wait();
+    if (rc == CRTB200_OK && rcs[i]) rc = fail(rcs[i], "device " + std::to_string(c->gpus[i]->device) + ": " + msgs[i]);
   }
   return rc;
 }
 
-static int upload_geometry_one(crtb200_ctx *c, const crtb200_scene *s, bool keep);
+// One multi-GPU pass over gpus[0..n): fn(i, gpu, stream) enqueues GPU i's part, GPU 0's on the caller's stream st and
+// every other GPU's on its own stream, which first waits for st's position.  on_workers: the other GPUs enqueue on
+// their helper threads (on_all_devices); otherwise they enqueue on the calling thread in order, up to the first that
+// fails.  st then waits for every GPU that started, also when a later one failed: what it enqueued writes into the
+// first GPU's memory.
+template <typename F>
+static int fan_out(crtb200_ctx *c, uint32_t n, cudaStream_t st, bool on_workers, F fn) {
+  CUDA_TRY(cudaSetDevice(c->gpus[0]->device));
+  if (n > 1) CUDA_TRY(cudaEventRecord(c->multi_fork, st));
+  std::vector<uint8_t> started(n, 0);
+  auto part = [&](size_t i, Gpu &g) -> int {
+    if (i == 0) return fn(0u, g, st);
+    CUDA_TRY(cudaSetDevice(g.device));
+    CUDA_TRY(cudaStreamWaitEvent(g.stream, c->multi_fork, 0));
+    started[i] = 1;
+    int rc = fn((uint32_t)i, g, (cudaStream_t)g.stream);
+    if (cudaEventRecord(g.multi_done, g.stream) != cudaSuccess && rc == CRTB200_OK) rc = fail(CRTB200_ERR_CUDA, "cudaEventRecord failed");
+    return rc;
+  };
+  int rc = CRTB200_OK;
+  if (on_workers)
+    rc = on_all_devices(c, part);
+  else
+    for (uint32_t i = 0; i < n && rc == CRTB200_OK; i++) rc = part(i, *c->gpus[i]);
+  CUDA_TRY(cudaSetDevice(c->gpus[0]->device));
+  for (uint32_t i = 1; i < n; i++)
+    if (started[i]) CUDA_TRY(cudaStreamWaitEvent(st, c->gpus[i]->multi_done, 0));
+  return rc;
+}
 
 extern "C" {
 
@@ -719,9 +768,8 @@ int crtb200_upload_scene(crtb200_ctx *c, const crtb200_scene *s) {
   c->trees_built = false;
   c->kd_nodes.release();
   c->kd_refs.release();
-  if (c->peers.empty()) return upload_one(c, s);
   // scene replicated on every GPU (SURVEY 8(e)); the host relayout runs once per GPU, in parallel
-  return on_all_devices(c, [&] { return upload_one(c, s); }, [&](size_t, crtb200_ctx *p) { return upload_one(p, s); });
+  return on_all_devices(c, [&](size_t, Gpu &g) { return upload_one(c, g, s); });
 }
 
 int crtb200_upload_geometry(crtb200_ctx *c, const crtb200_scene *s) {
@@ -735,9 +783,7 @@ int crtb200_upload_geometry(crtb200_ctx *c, const crtb200_scene *s) {
   c->kd_nodes.release();
   c->kd_refs.release();
   // one build per GPU, in parallel; only the first GPU keeps the reference-numbered trees for crtb200_scene_trees
-  const int rc = c->peers.empty() ? upload_geometry_one(c, s, true)
-                                  : on_all_devices(c, [&] { return upload_geometry_one(c, s, true); },
-                                                   [&](size_t, crtb200_ctx *p) { return upload_geometry_one(p, s, false); });
+  const int rc = on_all_devices(c, [&](size_t i, Gpu &g) { return upload_geometry_one(c, g, s, i == 0); });
   if (rc) {
     c->trees_built = false;
     c->kd_nodes.release();
@@ -761,8 +807,8 @@ struct SceneRecords {
 };
 
 // Validation and host records of the triangles, vertices, materials, textures and lights; `trees`: also check the
-// meshes' node and leaf-reference ranges (crtb200_upload_scene).  Selects the context's device and drops its scene.
-static int pack_records(crtb200_ctx *c, const crtb200_scene *s, bool trees, SceneRecords &r) {
+// meshes' node and leaf-reference ranges (crtb200_upload_scene).  Selects g's device and drops its scene.
+static int pack_records(Gpu &g, const crtb200_scene *s, bool trees, SceneRecords &r) {
   if (s->abi_version != CRTB200_ABI_VERSION) return fail(CRTB200_ERR_ARG, "crtb200_scene.abi_version mismatch");
   if (s->width == 0 || s->height == 0) return fail(CRTB200_ERR_SCENE, "image size is zero");
   if ((uint64_t)s->width * s->height > 0x7FFFFFFFull / 4) return fail(CRTB200_ERR_SCENE, "image too large");
@@ -772,8 +818,8 @@ static int pack_records(crtb200_ctx *c, const crtb200_scene *s, bool trees, Scen
       (s->n_mesh_leaf_refs && !s->mesh_leaf_refs) || (s->n_top_leaf_refs && !s->top_leaf_refs))
     return fail(CRTB200_ERR_SCENE, "a non-empty scene array is null");
   if (s->n_triangles >= 0x7FFFFFFFu || s->n_mesh_nodes >= 0x7FFFFFF0u) return fail(CRTB200_ERR_SCENE, "scene too large for 31-bit indices");
-  CUDA_TRY(cudaSetDevice(c->device));
-  c->have_scene = false;
+  CUDA_TRY(cudaSetDevice(g.device));
+  g.have_scene = false;
 
   // triangles
   r.geom.resize(3 * (size_t)s->n_triangles);
@@ -844,56 +890,55 @@ static int pack_records(crtb200_ctx *c, const crtb200_scene *s, bool trees, Scen
   return CRTB200_OK;
 }
 
-// The scene arena (nodes | leaf references | triangle geometry, one allocation, see crtb200_ctx::arena) for n_nodes
+// The scene arena (nodes | leaf references | triangle geometry, one allocation, see Gpu::arena) for n_nodes
 // nodes, n_refs mesh leaf references and the scene's triangles.
-static int place_arena(crtb200_ctx *c, size_t n_nodes, size_t n_refs, size_t n_geom) {
+static int place_arena(Gpu &g, size_t n_nodes, size_t n_refs, size_t n_geom) {
   auto al = [](size_t v) { return (v + 255) & ~(size_t)255; };
   const size_t b_nodes = al(n_nodes * 2 * sizeof(float4)), b_refs = al(n_refs * sizeof(uint32_t)), b_geom = al(n_geom * sizeof(float4));
-  c->arena_used = b_nodes + b_refs + b_geom;
-  c->nodes_bytes = b_nodes;
-  CUDA_TRY(c->arena.ensure(std::max<size_t>(c->arena_used, 256)));
-  c->nodes_p = reinterpret_cast<float4 *>(c->arena.p);
-  c->leaf_refs_p = reinterpret_cast<uint32_t *>(c->arena.p + b_nodes);
-  c->tri_geom_p = reinterpret_cast<float4 *>(c->arena.p + b_nodes + b_refs);
+  g.arena_used = b_nodes + b_refs + b_geom;
+  g.nodes_bytes = b_nodes;
+  CUDA_TRY(g.arena.ensure(std::max<size_t>(g.arena_used, 256)));
+  g.nodes_p = reinterpret_cast<float4 *>(g.arena.p);
+  g.leaf_refs_p = reinterpret_cast<uint32_t *>(g.arena.p + b_nodes);
+  g.tri_geom_p = reinterpret_cast<float4 *>(g.arena.p + b_nodes + b_refs);
   return CRTB200_OK;
 }
 
-// Uploads the records, sets the device scene and the frame buffers; the trees (arena nodes and references, top_refs,
-// meshes, nested_ok) are in place.
-static int commit_scene(crtb200_ctx *c, const crtb200_scene *s, const SceneRecords &r, uint32_t n_nodes, uint32_t n_refs,
+// Uploads the records to GPU g and sets its device scene, and on the context's first GPU the frame buffers; the trees
+// (arena nodes and references, top_refs, meshes, nested_ok) are in place.
+static int commit_scene(crtb200_ctx *c, Gpu &g, const crtb200_scene *s, const SceneRecords &r, uint32_t n_nodes, uint32_t n_refs,
                         uint32_t n_top_refs, uint32_t top_begin, uint32_t top_end) {
-  c->has_reflective = c->has_refractive = false;
+  g.has_reflective = g.has_refractive = false;
   for (uint32_t m = 0; m < s->n_meshes; m++) {
     const uint32_t type = s->materials[s->meshes[m].material].type;
-    if (type == CRTB200_MAT_REFLECTIVE) c->has_reflective = true;
-    if (type == CRTB200_MAT_REFRACTIVE) c->has_refractive = true;
+    if (type == CRTB200_MAT_REFLECTIVE) g.has_reflective = true;
+    if (type == CRTB200_MAT_REFRACTIVE) g.has_refractive = true;
   }
-  CUDA_TRY(c->tri_shade.upload(r.shade));
-  CUDA_TRY(c->vtx_normal.upload(r.vn));
-  if (!r.uv.empty()) CUDA_TRY(c->vtx_uv.upload(r.uv));
-  CUDA_TRY(c->materials.upload(r.mats));
-  CUDA_TRY(c->textures.upload(r.texs));
-  CUDA_TRY(c->texels.upload(r.texels));
-  CUDA_TRY(c->lights.upload(r.lights));
-  c->scene_bytes = (uint64_t)n_nodes * 32 + (uint64_t)n_refs * 4 + r.geom.size() * 16 + r.shade.size() * 16 + r.vn.size() * 16;
-  c->n_triangles = s->n_triangles;
-  c->n_nodes = n_nodes;
-  c->n_leaf_refs = n_refs;
-  c->n_top_refs = n_top_refs;
+  CUDA_TRY(g.tri_shade.upload(r.shade));
+  CUDA_TRY(g.vtx_normal.upload(r.vn));
+  if (!r.uv.empty()) CUDA_TRY(g.vtx_uv.upload(r.uv));
+  CUDA_TRY(g.materials.upload(r.mats));
+  CUDA_TRY(g.textures.upload(r.texs));
+  CUDA_TRY(g.texels.upload(r.texels));
+  CUDA_TRY(g.lights.upload(r.lights));
+  g.n_triangles = s->n_triangles;
+  g.n_nodes = n_nodes;
+  g.n_leaf_refs = n_refs;
+  g.n_top_refs = n_top_refs;
 
-  DScene &d = c->sc;
-  d.nodes = c->nodes_p;
-  d.leaf_refs = c->leaf_refs_p;
-  d.top_refs = c->top_refs.p;
-  d.tri_geom = c->tri_geom_p;
-  d.tri_shade = c->tri_shade.p;
-  d.vtx_normal = c->vtx_normal.p;
-  d.vtx_uv = r.uv.empty() ? nullptr : c->vtx_uv.p;
-  d.meshes = c->meshes.p;
-  d.materials = c->materials.p;
-  d.textures = c->textures.p;
-  d.texels = c->texels.p;
-  d.lights = c->lights.p;
+  DScene &d = g.sc;
+  d.nodes = g.nodes_p;
+  d.leaf_refs = g.leaf_refs_p;
+  d.top_refs = g.top_refs.p;
+  d.tri_geom = g.tri_geom_p;
+  d.tri_shade = g.tri_shade.p;
+  d.vtx_normal = g.vtx_normal.p;
+  d.vtx_uv = r.uv.empty() ? nullptr : g.vtx_uv.p;
+  d.meshes = g.meshes.p;
+  d.materials = g.materials.p;
+  d.textures = g.textures.p;
+  d.texels = g.texels.p;
+  d.lights = g.lights.p;
   d.n_lights = s->n_lights;
   d.n_meshes = s->n_meshes;
   d.top_begin = top_begin;
@@ -905,20 +950,22 @@ static int commit_scene(crtb200_ctx *c, const crtb200_scene *s, const SceneRecor
   d.dedup_words = d.dedup_meshes == 2u ? (s->n_meshes + 31u) / 32u : 0u;
 
   const size_t px = (size_t)s->width * s->height;
-  CUDA_TRY(c->frame.ensure(px * 3));
-  CUDA_TRY(cudaMemset(c->frame.p, 0, px * 3 * sizeof(float)));  // colorBuffer starts at (0,0,0), RayTracer.cpp:47-50
-  CUDA_TRY(c->frame8.ensure(px * 3));
-  CUDA_TRY(cudaMemset(c->frame8.p, 0, px * 3));
-  CUDA_TRY(c->stats_dev.ensure(CRT_STAT_SLOTS));
-  c->mask_valid = false;
-  c->cap_items = 0;
-  c->have_scene = true;
+  if (&g == c->gpus[0].get()) {
+    CUDA_TRY(c->frame.ensure(px * 3));
+    CUDA_TRY(cudaMemset(c->frame.p, 0, px * 3 * sizeof(float)));  // colorBuffer starts at (0,0,0), RayTracer.cpp:47-50
+    CUDA_TRY(c->frame8.ensure(px * 3));
+    CUDA_TRY(cudaMemset(c->frame8.p, 0, px * 3));
+  }
+  CUDA_TRY(g.stats_dev.ensure(CRT_STAT_SLOTS));
+  g.mask_valid = false;
+  g.cap_items = 0;
+  g.have_scene = true;
   return CRTB200_OK;
 }
 
-static int upload_one(crtb200_ctx *c, const crtb200_scene *s) {
+static int upload_one(crtb200_ctx *c, Gpu &g, const crtb200_scene *s) {
   SceneRecords r;
-  int rc = pack_records(c, s, true, r);
+  int rc = pack_records(g, s, true, r);
   if (rc) return rc;
   // trees: mesh trees first, top-level tree last, one node array
   std::vector<float4> nodes;
@@ -969,15 +1016,15 @@ static int upload_one(crtb200_ctx *c, const crtb200_scene *s) {
   for (uint32_t m = 0; m < s->n_meshes; m++) meshes[m].cull_margin = mesh_cull_margin(s, s->meshes[m], nested_ok);
   std::vector<uint32_t> top_refs(s->top_leaf_refs, s->top_leaf_refs + s->n_top_leaf_refs);
 
-  rc = place_arena(c, nodes.size() / 2, refs.size(), r.geom.size());
+  rc = place_arena(g, nodes.size() / 2, refs.size(), r.geom.size());
   if (rc) return rc;
-  if (!nodes.empty()) CUDA_TRY(cudaMemcpy(c->nodes_p, nodes.data(), nodes.size() * sizeof(float4), cudaMemcpyHostToDevice));
-  if (!refs.empty()) CUDA_TRY(cudaMemcpy(c->leaf_refs_p, refs.data(), refs.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
-  if (!r.geom.empty()) CUDA_TRY(cudaMemcpy(c->tri_geom_p, r.geom.data(), r.geom.size() * sizeof(float4), cudaMemcpyHostToDevice));
-  c->nested_ok = nested_ok;
-  CUDA_TRY(c->top_refs.upload(top_refs));
-  CUDA_TRY(c->meshes.upload(meshes));
-  return commit_scene(c, s, r, (uint32_t)(nodes.size() / 2), (uint32_t)refs.size(), (uint32_t)top_refs.size(), top_begin, top_end);
+  if (!nodes.empty()) CUDA_TRY(cudaMemcpy(g.nodes_p, nodes.data(), nodes.size() * sizeof(float4), cudaMemcpyHostToDevice));
+  if (!refs.empty()) CUDA_TRY(cudaMemcpy(g.leaf_refs_p, refs.data(), refs.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
+  if (!r.geom.empty()) CUDA_TRY(cudaMemcpy(g.tri_geom_p, r.geom.data(), r.geom.size() * sizeof(float4), cudaMemcpyHostToDevice));
+  g.nested_ok = nested_ok;
+  CUDA_TRY(g.top_refs.upload(top_refs));
+  CUDA_TRY(g.meshes.upload(meshes));
+  return commit_scene(c, g, s, r, (uint32_t)(nodes.size() / 2), (uint32_t)refs.size(), (uint32_t)top_refs.size(), top_begin, top_end);
 }
 
 // ---- device KD build: crtb200_upload_geometry (csrc/crt_build.cuh, DESIGN.md 3.11) -------------------------------
@@ -1034,11 +1081,11 @@ struct BuildAdd4 {
 
 static unsigned build_blocks(uint64_t n) { return (unsigned)std::max<uint64_t>(1, (n + 255) / 256); }
 
-// Builds the trees of `s` on c's GPU and uploads the scene; keep: also keep the reference-numbered trees for
+// Builds the trees of `s` on GPU g of context c and uploads the scene; keep: also keep the reference-numbered trees for
 // crtb200_scene_trees.
-static int upload_geometry_one(crtb200_ctx *c, const crtb200_scene *s, bool keep) {
+static int upload_geometry_one(crtb200_ctx *c, Gpu &g, const crtb200_scene *s, bool keep) {
   SceneRecords r;
-  int rc = pack_records(c, s, false, r);
+  int rc = pack_records(g, s, false, r);
   if (rc) return rc;
   const uint32_t M = s->n_meshes, T = M + 1;
   std::vector<uint32_t> item_base(M + 1), mesh_tri(std::max(M, 1u), 0);
@@ -1051,13 +1098,13 @@ static int upload_geometry_one(crtb200_ctx *c, const crtb200_scene *s, bool keep
   if (items + M >= 0x7FFFFFFFull) return fail(CRTB200_ERR_SCENE, "scene too large for 31-bit indices");
   item_base[M] = (uint32_t)items;
   const uint32_t NI = (uint32_t)items, NE = NI + M;
-  cudaStream_t st = c->stream;
+  cudaStream_t st = g.stream;
 
   BuildScratch sc;
   bool ok = true;
   auto al = [&](auto *&p, size_t n) { ok = ok && sc.alloc(p, n); };
   auto nomem = [&]() {
-    return fail(CRTB200_ERR_MEMORY, "device KD build: scratch does not fit on device " + std::to_string(c->device) + " (" +
+    return fail(CRTB200_ERR_MEMORY, "device KD build: scratch does not fit on device " + std::to_string(g.device) + " (" +
                                         std::to_string(sc.live) + " bytes allocated)");
   };
   float4 *geom;
@@ -1214,10 +1261,10 @@ static int upload_geometry_one(crtb200_ctx *c, const crtb200_scene *s, bool keep
 
   // the scene's device arrays: arena, top-level references, meshes (the margins follow), kept trees
   CUDA_TRY(cudaStreamSynchronize(st));
-  rc = place_arena(c, n_nodes, n_refs, r.geom.size());
+  rc = place_arena(g, n_nodes, n_refs, r.geom.size());
   if (rc) return rc;
-  if (!r.geom.empty()) CUDA_TRY(cudaMemcpyAsync(c->tri_geom_p, geom, r.geom.size() * sizeof(float4), cudaMemcpyDeviceToDevice, st));
-  CUDA_TRY(c->top_refs.ensure(std::max<uint32_t>(n_top_refs, 1)));
+  if (!r.geom.empty()) CUDA_TRY(cudaMemcpyAsync(g.tri_geom_p, geom, r.geom.size() * sizeof(float4), cudaMemcpyDeviceToDevice, st));
+  CUDA_TRY(g.top_refs.ensure(std::max<uint32_t>(n_top_refs, 1)));
   std::vector<DMesh> meshes(M);
   for (uint32_t m = 0; m < M; m++) {
     meshes[m].node_begin = node_base[m];
@@ -1226,11 +1273,11 @@ static int upload_geometry_one(crtb200_ctx *c, const crtb200_scene *s, bool keep
     meshes[m].first_triangle = s->meshes[m].first_triangle;
     meshes[m].cull_margin = std::numeric_limits<float>::infinity();
   }
-  CUDA_TRY(c->meshes.upload(meshes));
+  CUDA_TRY(g.meshes.upload(meshes));
   if (keep) {
     if (c->kd_nodes.ensure(std::max<uint64_t>(n_nodes, 1)) != cudaSuccess || c->kd_refs.ensure(std::max<uint64_t>(n_refs, 1)) != cudaSuccess) {
       cudaGetLastError();
-      return fail(CRTB200_ERR_MEMORY, "device KD build: the built trees do not fit on device " + std::to_string(c->device));
+      return fail(CRTB200_ERR_MEMORY, "device KD build: the built trees do not fit on device " + std::to_string(g.device));
     }
   }
   for (uint32_t l = 0; l < D; l++) {
@@ -1238,11 +1285,11 @@ static int upload_geometry_one(crtb200_ctx *c, const crtb200_scene *s, bool keep
     const BuildLevel *N = l + 1 < D ? &lv[l + 1] : nullptr;
     k_build_write<<<build_blocks(L.n), 256, 0, st>>>(L.nodes, L.n, M, NI, L.child, L.leaf_cnt, L.leaf_off, L.leafbuf, L.size, L.pre, L.vis,
                                                      L.ref, N ? N->pre : nullptr, N ? N->vis : nullptr, d_node_base, d_ref_base,
-                                                     d_item_base, d_mesh_tri, geom, c->nodes_p, c->leaf_refs_p, c->top_refs.p,
+                                                     d_item_base, d_mesh_tri, geom, g.nodes_p, g.leaf_refs_p, g.top_refs.p,
                                                      keep ? c->kd_nodes.p : nullptr, keep ? c->kd_refs.p : nullptr, slots);
   }
   if (NI) k_build_tri_margin<<<build_blocks(NI), 256, 0, st>>>(geom, d_item_base, d_mesh_tri, M, NI, slots);
-  if (M) k_build_margins<<<build_blocks(M), 256, 0, st>>>(M, slots, nested, c->meshes.p);
+  if (M) k_build_margins<<<build_blocks(M), 256, 0, st>>>(M, slots, nested, g.meshes.p);
   CUDA_TRY(cudaGetLastError());
   CUDA_TRY(cudaEventRecord(ev1, st));
   uint32_t nested_h = 0;
@@ -1250,7 +1297,7 @@ static int upload_geometry_one(crtb200_ctx *c, const crtb200_scene *s, bool keep
   CUDA_TRY(cudaStreamSynchronize(st));
   float build_ms = 0.f;
   cudaEventElapsedTime(&build_ms, ev0, ev1);
-  c->nested_ok = nested_h != 0;  // every tree is at most 26 levels deep: k_coop's limit of 40 always holds
+  g.nested_ok = nested_h != 0;  // every tree is at most 26 levels deep: k_coop's limit of 40 always holds
 
   if (keep) {
     c->kd_meshes.assign(s->meshes, s->meshes + M);
@@ -1270,7 +1317,7 @@ static int upload_geometry_one(crtb200_ctx *c, const crtb200_scene *s, bool keep
     k.peak_scratch_bytes = sc.peak;
     k.build_ms = build_ms;
   }
-  rc = commit_scene(c, s, r, (uint32_t)n_nodes, (uint32_t)n_refs, n_top_refs, top_begin, (uint32_t)n_nodes);
+  rc = commit_scene(c, g, s, r, (uint32_t)n_nodes, (uint32_t)n_refs, n_top_refs, top_begin, (uint32_t)n_nodes);
   if (rc == CRTB200_OK && keep) c->trees_built = true;
   return rc;
 }
@@ -1278,15 +1325,15 @@ static int upload_geometry_one(crtb200_ctx *c, const crtb200_scene *s, bool keep
 // ---- frame planning ------------------------------------------------------------------------------------------
 // worst-case children of one ray-tree node: refractive hits spawn two (RayTracer.cpp:398-412), reflective ones one, and
 // in GI frames diffuse hits G (crtb200_sampling.gi_samples)
-static uint32_t node_branching(const crtb200_ctx *c) {
-  uint32_t b = c->has_refractive ? 2u : (c->has_reflective ? 1u : 0u);
-  if (c->sampling.use_gi) b = std::max(b, c->sampling.gi_samples);
+static uint32_t node_branching(const Gpu &g, const crtb200_sampling &smp) {
+  uint32_t b = g.has_refractive ? 2u : (g.has_reflective ? 1u : 0u);
+  if (smp.use_gi) b = std::max(b, smp.gi_samples);
   return b;
 }
 
-static uint32_t branching_sum(const crtb200_ctx *c, uint32_t max_depth, uint64_t *per_level) {
+static uint32_t branching_sum(const Gpu &g, const crtb200_sampling &smp, uint32_t max_depth, uint64_t *per_level) {
   // worst-case rays per level-0 item at each level: branching^level, saturated at 2^40 (far beyond any queue budget)
-  const uint64_t branch = node_branching(c), cap = 1ull << 40;
+  const uint64_t branch = node_branching(g, smp), cap = 1ull << 40;
   uint64_t sum = 0, b = 1;
   for (uint32_t l = 0; l <= max_depth; l++) {
     per_level[l] = b;
@@ -1298,25 +1345,27 @@ static uint32_t branching_sum(const crtb200_ctx *c, uint32_t max_depth, uint64_t
 
 // Marks the scene arena as L2-persisting for the kernels of `st` (one access-policy window per stream).  When the arena
 // is larger than the persisting carve-out, hitRatio makes a matching fraction of its lines persist instead of thrashing.
-static void apply_l2_window(crtb200_ctx *c, cudaStream_t st) {
-  if (!c->l2_persist || !c->l2_persist_max || !c->l2_window_max || !c->arena_used) return;
+static void apply_l2_window(const Gpu &g, cudaStream_t st) {
+  if (!g.l2_persist || !g.l2_persist_max || !g.l2_window_max || !g.arena_used) return;
   cudaStreamAttrValue v{};
-  const size_t bytes = std::min(c->l2_persist == 3 ? c->nodes_bytes : c->arena_used, c->l2_window_max);
-  v.accessPolicyWindow.base_ptr = c->arena.p;
+  const size_t bytes = std::min(g.l2_persist == 3 ? g.nodes_bytes : g.arena_used, g.l2_window_max);
+  v.accessPolicyWindow.base_ptr = g.arena.p;
   v.accessPolicyWindow.num_bytes = bytes;
-  v.accessPolicyWindow.hitRatio = (float)std::min(1.0, (double)c->l2_persist_max / (double)bytes);
+  v.accessPolicyWindow.hitRatio = (float)std::min(1.0, (double)g.l2_persist_max / (double)bytes);
   v.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-  v.accessPolicyWindow.missProp = c->l2_persist == 1 ? cudaAccessPropertyStreaming : cudaAccessPropertyNormal;
+  v.accessPolicyWindow.missProp = g.l2_persist == 1 ? cudaAccessPropertyStreaming : cudaAccessPropertyNormal;
   cudaStreamSetAttribute(st, cudaStreamAttributeAccessPolicyWindow, &v);
   cudaGetLastError();  // a hint: never an error of the render
 }
 
-static int plan_queues(crtb200_ctx *c, uint32_t shard_items, uint32_t max_depth, uint32_t row_items, bool pipelined) {
+// Queues of GPU g for a frame with sampling smp, under the context's queue budget and concurrency
+static int plan_queues(const crtb200_ctx *c, Gpu &g, const crtb200_sampling &smp, uint32_t shard_items, uint32_t max_depth,
+                       uint32_t row_items, bool pipelined) {
   uint64_t per_level[CRT_MAX_LEVELS] = {0};
-  branching_sum(c, max_depth, per_level);
+  branching_sum(g, smp, max_depth, per_level);
   uint64_t sum = 0;
   for (uint32_t l = 0; l <= max_depth; l++) sum += per_level[l];
-  const uint32_t n_lights = std::max<uint32_t>(1, c->sc.n_lights);
+  const uint32_t n_lights = std::max<uint32_t>(1, g.sc.n_lights);
   const uint64_t bytes_per_node = 32 + 8 + 16 + 16 + 48 + n_lights;  // ray + hit + colour + comb + diffuse item + visibility bytes
   // sets used: up to `concurrency`, but never chunks smaller than 64 Ki items (launch overhead would dominate)
   uint32_t n_sets = std::max<uint32_t>(1, std::min<uint32_t>(c->concurrency, (shard_items + 65535u) / 65536u));
@@ -1331,7 +1380,7 @@ static int plan_queues(crtb200_ctx *c, uint32_t shard_items, uint32_t max_depth,
   uint64_t items = c->queue_budget / (bytes_per_node * sum * n_sets);
   items &= ~31ull;
   if (items < 32 * 64)
-    return fail(CRTB200_ERR_MEMORY, c->sampling.use_gi ? "queue budget too small for one chunk of 2048 pixels: the GI ray tree has up to "
+    return fail(CRTB200_ERR_MEMORY, smp.use_gi ? "queue budget too small for one chunk of 2048 pixels: the GI ray tree has up to "
                                                              "gi_samples^max_depth nodes per pixel; lower gi_samples or max_depth"
                                                        : "queue budget too small for one chunk at this ray depth");
   // host-bound frames: one chunk per stream at 1080p, two at 4K (a band's copy overlaps the traversal of the next band;
@@ -1346,14 +1395,14 @@ static int plan_queues(crtb200_ctx *c, uint32_t shard_items, uint32_t max_depth,
   if (items * sum * n_lights >= 0x7FFFFFFFull) items = ((0x7FFFFFFFull / (sum * n_lights)) - 32) & ~31ull;
   if (items < 32) return fail(CRTB200_ERR_MEMORY, "too many lights x ray-tree nodes for 32-bit queue slots");
   if (items >= row_items) items = (items / row_items) * row_items;  // whole tile rows (band copies need it)
-  c->n_chunks = (uint32_t)((shard_items + items - 1) / items);
-  if (c->cap_items == items && c->cap_depth == max_depth && c->cap_sets == n_sets && c->cap_branch == node_branching(c)) return CRTB200_OK;
-  if (c->sets.size() < n_sets) c->sets.resize(n_sets);
-  CUDA_TRY(c->fork_ev.create(cudaEventDisableTiming));
+  g.n_chunks = (uint32_t)((shard_items + items - 1) / items);
+  if (g.cap_items == items && g.cap_depth == max_depth && g.cap_sets == n_sets && g.cap_branch == node_branching(g, smp)) return CRTB200_OK;
+  if (g.sets.size() < n_sets) g.sets.resize(n_sets);
+  CUDA_TRY(g.fork_ev.create(cudaEventDisableTiming));
   for (uint32_t k = 0; k < n_sets; k++) {
-    crtb200_ctx::QueueSet &q = c->sets[k];
+    QueueSet &q = g.sets[k];
     CUDA_TRY(q.stream.create(cudaStreamNonBlocking));
-    apply_l2_window(c, q.stream);
+    apply_l2_window(g, q.stream);
     CUDA_TRY(q.done.create(cudaEventDisableTiming));
     uint64_t total = 0;
     for (uint32_t l = 0; l <= max_depth; l++) {
@@ -1369,9 +1418,9 @@ static int plan_queues(crtb200_ctx *c, uint32_t shard_items, uint32_t max_depth,
     CUDA_TRY(q.color.ensure(total));
     CUDA_TRY(q.comb.ensure(total));
     CUDA_TRY(q.dq.ensure(3 * total));
-    CUDA_TRY(q.vis.ensure(std::max<uint64_t>(1, total * std::max<uint32_t>(1, c->sc.n_lights))));
+    CUDA_TRY(q.vis.ensure(std::max<uint64_t>(1, total * std::max<uint32_t>(1, g.sc.n_lights))));
     // hand-off records: every lane of a traversal grid hands off at most once per launch
-    const uint64_t ovf_cap = (uint64_t)std::max(c->blocks_closest, c->blocks_shadow) * CRT_TRAV_BLOCK;
+    const uint64_t ovf_cap = (uint64_t)std::max(g.blocks_closest, g.blocks_shadow) * CRT_TRAV_BLOCK;
     CUDA_TRY(q.ovf.ensure(3 * ovf_cap));
     // every record starts out "not published" (r0.x = CRT_INVALID); k_coop leaves a taken record in that state again
     CUDA_TRY(cudaMemsetAsync(q.ovf.p, 0xFF, 3 * ovf_cap * sizeof(uint4), q.stream));
@@ -1386,7 +1435,7 @@ static int plan_queues(crtb200_ctx *c, uint32_t shard_items, uint32_t max_depth,
     q.work = q.ctl.p + n_counts;
     q.lv.ovf = q.ovf.p;
     q.lv.ovf_ctl = q.ctl.p + n_counts + n_work;
-    q.lv.ovf_cap = (uint32_t)std::min<uint64_t>(ovf_cap, (uint64_t)c->tail_cap * c->blocks_coop * CRT_COOP_WARPS);
+    q.lv.ovf_cap = (uint32_t)std::min<uint64_t>(ovf_cap, (uint64_t)g.tail_cap * g.blocks_coop * CRT_COOP_WARPS);
     q.lv.tail_iters = 0;
     q.lv.tail_start = 512;
     q.lv.tail_start_closest = 256;
@@ -1401,12 +1450,12 @@ static int plan_queues(crtb200_ctx *c, uint32_t shard_items, uint32_t max_depth,
     q.lv.dq = q.dq.p;
     q.lv.vis = q.vis.p;
     q.lv.counts = q.ctl.p;
-    q.lv.stats = c->stats_dev.p;
+    q.lv.stats = g.stats_dev.p;
   }
-  c->cap_items = (uint32_t)items;
-  c->cap_depth = max_depth;
-  c->cap_sets = n_sets;
-  c->cap_branch = node_branching(c);
+  g.cap_items = (uint32_t)items;
+  g.cap_depth = max_depth;
+  g.cap_sets = n_sets;
+  g.cap_branch = node_branching(g, smp);
   return CRTB200_OK;
 }
 
@@ -1424,23 +1473,23 @@ static size_t rect_coverage(uint32_t W, uint32_t H, const std::vector<crtb200_re
   return covered;
 }
 
-static int plan_mask(crtb200_ctx *c, const crtb200_options *o) {
-  const uint32_t W = c->sc.width, H = c->sc.height;
+static int plan_mask(Gpu &g, const crtb200_options *o) {
+  const uint32_t W = g.sc.width, H = g.sc.height;
   std::vector<crtb200_rect> rects(o->rects, o->rects + o->n_rects);
-  if (c->mask_valid && rects.size() == c->mask_rects.size() &&
-      (rects.empty() || !std::memcmp(rects.data(), c->mask_rects.data(), rects.size() * sizeof(crtb200_rect))))
+  if (g.mask_valid && rects.size() == g.mask_rects.size() &&
+      (rects.empty() || !std::memcmp(rects.data(), g.mask_rects.data(), rects.size() * sizeof(crtb200_rect))))
     return CRTB200_OK;
-  c->mask_rects = rects;
-  c->mask_needed = false;
+  g.mask_rects = rects;
+  g.mask_needed = false;
   if (!rects.empty()) {
     std::vector<uint8_t> m;
     if (rect_coverage(W, H, rects, m) != m.size()) {
-      c->mask_needed = true;
-      CUDA_TRY(c->mask.ensure(m.size()));
-      CUDA_TRY(cudaMemcpy(c->mask.p, m.data(), m.size(), cudaMemcpyHostToDevice));
+      g.mask_needed = true;
+      CUDA_TRY(g.mask.ensure(m.size()));
+      CUDA_TRY(cudaMemcpy(g.mask.p, m.data(), m.size(), cudaMemcpyHostToDevice));
     }
   }
-  c->mask_valid = true;
+  g.mask_valid = true;
   return CRTB200_OK;
 }
 
@@ -1453,16 +1502,16 @@ static cudaError_t record_next_event(crtb200_ctx *c, cudaStream_t st) {
 }
 
 // dynamic shared memory of the kernels that walk one ray per lane: the visited-mesh bitset of scenes with > 64 meshes
-static size_t dyn_smem(const crtb200_ctx *c, int block) { return (size_t)c->sc.dedup_words * (size_t)block * sizeof(uint32_t); }
+static size_t dyn_smem(const Gpu &g, int block) { return (size_t)g.sc.dedup_words * (size_t)block * sizeof(uint32_t); }
 
-// A caller's device pointer: device memory of the context's first GPU, `align`-byte aligned
-static int check_device_ptr(const crtb200_ctx *c, const void *p, size_t align, const char *what) {
+// A caller's device pointer: device memory of the context's first GPU g, `align`-byte aligned
+static int check_device_ptr(const Gpu &g, const void *p, size_t align, const char *what) {
   if (!p) return fail(CRTB200_ERR_ARG, std::string(what) + " is null");
   if (reinterpret_cast<uintptr_t>(p) % align) return fail(CRTB200_ERR_ARG, std::string(what) + " is not " + std::to_string(align) + "-byte aligned");
   cudaPointerAttributes a{};
   const cudaError_t e = cudaPointerGetAttributes(&a, p);
   if (e != cudaSuccess) cudaGetLastError();  // (not a CUDA pointer: not sticky)
-  if (e != cudaSuccess || a.type != cudaMemoryTypeDevice || a.device != c->device)
+  if (e != cudaSuccess || a.type != cudaMemoryTypeDevice || a.device != g.device)
     return fail(CRTB200_ERR_ARG, std::string(what) + " is not device memory of the context's first GPU");
   return CRTB200_OK;
 }
@@ -1476,25 +1525,23 @@ struct Flavour {
   bool cull, handoff, gi, wide_closest, wide_shadow;
 };
 
-static Flavour frame_flavour(const crtb200_ctx *c, const crtb200_options *o) {
-  const bool wide = c->sc.dedup_meshes == 2u;
+static Flavour frame_flavour(const Gpu &g, const crtb200_options *o, const crtb200_sampling &smp) {
+  const bool wide = g.sc.dedup_meshes == 2u;
   return Flavour{o->count_work,
-                 o->traversal == 0 && o->count_work != 1 && c->nested_ok,
-                 o->traversal == 0 && o->count_work == 0 && c->nested_ok && c->tail_iters >= 0,
-                 c->sampling.use_gi != 0,
+                 o->traversal == 0 && o->count_work != 1 && g.nested_ok,
+                 o->traversal == 0 && o->count_work == 0 && g.nested_ok && g.tail_iters >= 0,
+                 smp.use_gi != 0,
                  o->count_work == 0 && wide,
                  o->count_work != 1 && wide};
 }
 
 // The kernel flavours of a caller's ray batch (crtb200_trace_rays_device): a frame's with the batch's traversal and
 // count_work -- literal walk without hand-off for traversal 1, count_work 1 and trees that do not nest -- never GI.
-static Flavour query_flavour(const crtb200_ctx *c, const crtb200_ray_batch *b) {
+static Flavour query_flavour(const Gpu &g, const crtb200_ray_batch *b) {
   crtb200_options o{};
   o.traversal = b->traversal;
   o.count_work = b->count_work;
-  Flavour fl = frame_flavour(c, &o);
-  fl.gi = false;
-  return fl;
+  return frame_flavour(g, &o, crtb200_sampling{});
 }
 
 // f(v) with v as a compile-time constant: how the launch functions below turn a Flavour into template arguments
@@ -1506,33 +1553,33 @@ static void as_const_count(uint32_t v, F &&f) {
 }
 
 // k_closest of level `level`: PRIMARY at level 0, jittered in GI frames
-static void launch_closest(crtb200_ctx *c, const Flavour &fl, const Frame &fr, crtb200_ctx::QueueSet &q, uint32_t level) {
+static void launch_closest(const Gpu &g, const Flavour &fl, const Frame &fr, QueueSet &q, uint32_t level) {
   const bool primary = level == 0;
   as_const(fl.count_work != 0, [&](auto count) { as_const(fl.cull, [&](auto cull) { as_const(fl.wide_closest, [&](auto wide) {
     as_const(primary, [&](auto prim) { as_const(primary && fl.gi, [&](auto jitter) {
       if constexpr (!(count && wide) && (prim || !jitter))
         k_closest<prim, count, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, cull, wide, jitter>
-            <<<primary ? c->blocks_closest : c->blocks_closest_sec, CRT_TRAV_BLOCK, dyn_smem(c, CRT_TRAV_BLOCK), q.stream>>>(
-                c->sc, fr, q.lv, level, q.work + CRT_CTL_STRIDE * level);
+            <<<primary ? g.blocks_closest : g.blocks_closest_sec, CRT_TRAV_BLOCK, dyn_smem(g, CRT_TRAV_BLOCK), q.stream>>>(
+                g.sc, fr, q.lv, level, q.work + CRT_CTL_STRIDE * level);
     }); }); }); }); });
 }
 // the shadow pass of one chunk; SKIPR = false in GI frames
-static void launch_shadow(crtb200_ctx *c, const Flavour &fl, const Frame &fr, crtb200_ctx::QueueSet &q) {
+static void launch_shadow(const Gpu &g, const Flavour &fl, const Frame &fr, QueueSet &q) {
   as_const_count(fl.count_work, [&](auto count) { as_const(fl.cull, [&](auto cull) { as_const(fl.wide_shadow, [&](auto wide) {
     as_const(!fl.gi, [&](auto skipr) {
       if constexpr (count != 1 || !(cull || wide))
         k_shadow<count, CRT_REFILL_SHADOW, CRT_LOOP_MODE, cull, wide, skipr>
-            <<<c->blocks_shadow, CRT_TRAV_BLOCK, wide ? dyn_smem(c, CRT_TRAV_BLOCK) : 0, q.stream>>>(
-                c->sc, fr, q.lv, q.work + CRT_CTL_STRIDE * CRT_MAX_LEVELS);
+            <<<g.blocks_shadow, CRT_TRAV_BLOCK, wide ? dyn_smem(g, CRT_TRAV_BLOCK) : 0, q.stream>>>(
+                g.sc, fr, q.lv, q.work + CRT_CTL_STRIDE * CRT_MAX_LEVELS);
     }); }); }); });
 }
 // k_coop over the walks the shadow pass or closest-hit level `level` handed off; SKIPR = false in GI shadow passes
-static void launch_coop(crtb200_ctx *c, const Flavour &fl, const Frame &fr, crtb200_ctx::QueueSet &q, bool shadow, uint32_t level,
+static void launch_coop(const Gpu &g, const Flavour &fl, const Frame &fr, QueueSet &q, bool shadow, uint32_t level,
                         int blocks, cudaStream_t st, uint32_t early) {
   as_const(shadow, [&](auto sh) { as_const(!shadow && level == 0, [&](auto prim) { as_const(fl.cull, [&](auto cull) {
     as_const(!(shadow && fl.gi), [&](auto skipr) {
       if constexpr (!(sh && prim) && (sh || skipr))
-        k_coop<sh, prim, cull, CRT_COOP_GROUP, skipr><<<blocks, 32 * CRT_COOP_WARPS, 0, st>>>(c->sc, fr, q.lv, level, early);
+        k_coop<sh, prim, cull, CRT_COOP_GROUP, skipr><<<blocks, 32 * CRT_COOP_WARPS, 0, st>>>(g.sc, fr, q.lv, level, early);
     }); }); }); });
 }
 
@@ -1542,16 +1589,17 @@ static void launch_coop(crtb200_ctx *c, const Flavour &fl, const Frame &fr, crtb
 // frame) the side stream is forked BEFORE the traversal kernel is launched; behind it k_mark marks the traversal kernel's
 // end, the early pass starts on the side stream (its blocks get SM resources as the traversal kernel's blocks exit)
 // and joins, and the final pass runs over what is left.
-// per_kernel: time them (closest_ms, shadow_ms, coop_*_ms); a mark with a kind (0 closest, 1 shadow, 2 / 3 their k_coop
-// part) opens a span and the next mark closes it, collect_stats_one reads them in pairs.
+// timed: the context whose per-launch events time them (closest_ms, shadow_ms, coop_*_ms), null for none; a mark with a
+// kind (0 closest, 1 shadow, 2 / 3 their k_coop part) opens a span and the next mark closes it, collect_stats reads
+// them in pairs.
 template <typename Launch>
-static int traverse(crtb200_ctx *c, bool handoff, bool early_ok, crtb200_ctx::QueueSet &q, cudaStream_t st, bool shadow,
-                    uint32_t level, bool per_kernel, uint32_t &launches, const Launch &launch) {
+static int traverse(Gpu &g, bool handoff, bool early_ok, QueueSet &q, cudaStream_t st, bool shadow, uint32_t level,
+                    crtb200_ctx *timed, uint32_t &launches, const Launch &launch) {
   auto mark = [&](int kind) {
-    if (per_kernel && kind >= 0) c->kev_kind.push_back(kind);
-    return per_kernel ? record_next_event(c, st) : cudaSuccess;
+    if (timed && kind >= 0) timed->kev_kind.push_back(kind);
+    return timed ? record_next_event(timed, st) : cudaSuccess;
   };
-  const bool early = handoff && c->coop_early > 0 && early_ok;
+  const bool early = handoff && g.coop_early > 0 && early_ok;
   CUDA_TRY(mark(shadow ? 1 : 0));
   if (early) {
     CUDA_TRY(cudaEventRecord(q.coop_fork, st));
@@ -1563,12 +1611,12 @@ static int traverse(crtb200_ctx *c, bool handoff, bool early_ok, crtb200_ctx::Qu
     CUDA_TRY(mark(shadow ? 3 : 2));
     if (early) {
       k_mark<<<1, 32, 0, st>>>(q.lv.ovf_ctl + CRT_CTL_STRIDE * (shadow ? (uint32_t)CRT_MAX_LEVELS : level) + 24u);
-      launch(q.coop_stream, c->sm_count * c->coop_early, 1u);
+      launch(q.coop_stream, g.sm_count * g.coop_early, 1u);
       CUDA_TRY(cudaEventRecord(q.coop_join, q.coop_stream));
       CUDA_TRY(cudaStreamWaitEvent(st, q.coop_join, 0));
       launches += 2;
     }
-    launch(st, c->blocks_coop, 0u);
+    launch(st, g.blocks_coop, 0u);
     launches++;
   }
   CUDA_TRY(mark(-1));
@@ -1576,51 +1624,51 @@ static int traverse(crtb200_ctx *c, bool handoff, bool early_ok, crtb200_ctx::Qu
 }
 
 // traverse for k_closest of level `level` or the shadow pass of a frame's chunk
-static int traverse_frame(crtb200_ctx *c, const Flavour &fl, const Frame &fr, crtb200_ctx::QueueSet &q, bool shadow, uint32_t level,
-                          bool per_kernel, uint32_t &launches) {
-  return traverse(c, fl.handoff, c->cap_sets == 1 && (shadow || level == 0), q, q.stream, shadow, level, per_kernel, launches,
+static int traverse_frame(Gpu &g, const Flavour &fl, const Frame &fr, QueueSet &q, bool shadow, uint32_t level,
+                          crtb200_ctx *timed, uint32_t &launches) {
+  return traverse(g, fl.handoff, g.cap_sets == 1 && (shadow || level == 0), q, q.stream, shadow, level, timed, launches,
                   [&](cudaStream_t st, int coop_blocks, uint32_t early) {
                     if (coop_blocks)
-                      launch_coop(c, fl, fr, q, shadow, level, coop_blocks, st, early);
+                      launch_coop(g, fl, fr, q, shadow, level, coop_blocks, st, early);
                     else if (shadow)
-                      launch_shadow(c, fl, fr, q);
+                      launch_shadow(g, fl, fr, q);
                     else
-                      launch_closest(c, fl, fr, q, level);
+                      launch_closest(g, fl, fr, q, level);
                   });
 }
 
 // One query batch `qb` on GPU x (its range of a multi-GPU batch) on stream st: the query's counters zeroed, the query
 // kernel of the ray type and, with hand-off, k_coop_query around it (traverse).  Closest hits use the work cursor and
 // hand-off line of launch 0, shadow queries those of launch CRT_MAX_LEVELS, as k_coop_query reads them.
-static int enqueue_query(crtb200_ctx *x, const Flavour &fl, uint32_t ray_type, const QueryBatch &qb, cudaStream_t st,
+static int enqueue_query(Gpu &x, const Flavour &fl, uint32_t ray_type, const QueryBatch &qb, cudaStream_t st,
                          uint32_t &launches) {
-  crtb200_ctx::QueueSet &q = x->query;
-  q.lv.tail_iters = fl.handoff ? (uint32_t)(x->tail_iters + 1) : 0u;
-  q.lv.tail_start = (uint32_t)x->tail_start;
-  q.lv.tail_start_closest = (uint32_t)x->tail_start_closest;
-  q.lv.tail_small = (uint32_t)x->tail_small;
+  QueueSet &q = x.query;
+  q.lv.tail_iters = fl.handoff ? (uint32_t)(x.tail_iters + 1) : 0u;
+  q.lv.tail_start = (uint32_t)x.tail_start;
+  q.lv.tail_start_closest = (uint32_t)x.tail_start_closest;
+  q.lv.tail_small = (uint32_t)x.tail_small;
   CUDA_TRY(cudaMemsetAsync(q.ctl.p, 0, q.ctl.n * sizeof(uint32_t), st));
-  CUDA_TRY(cudaMemsetAsync(x->query_stats_dev.p, 0, CRT_STAT_SLOTS * sizeof(unsigned long long), st));
+  CUDA_TRY(cudaMemsetAsync(x.query_stats_dev.p, 0, CRT_STAT_SLOTS * sizeof(unsigned long long), st));
   const bool shadow = ray_type == CRTB200_RAY_SHADOW, primary = ray_type == CRTB200_RAY_PRIMARY;
   uint32_t *const work = q.work + CRT_CTL_STRIDE * (shadow ? (uint32_t)CRT_MAX_LEVELS : 0u);
   launches++;
-  return traverse(x, fl.handoff, true, q, st, shadow, 0, false, launches, [&](cudaStream_t s, int coop_blocks, uint32_t early) {
+  return traverse(x, fl.handoff, true, q, st, shadow, 0, nullptr, launches, [&](cudaStream_t s, int coop_blocks, uint32_t early) {
     if (coop_blocks) {
       as_const(shadow, [&](auto sh) { as_const(primary, [&](auto prim) {
-        if constexpr (!(sh && prim)) k_coop_query<sh, prim><<<coop_blocks, 32 * CRT_COOP_WARPS, 0, s>>>(x->sc, q.lv, qb, early);
+        if constexpr (!(sh && prim)) k_coop_query<sh, prim><<<coop_blocks, 32 * CRT_COOP_WARPS, 0, s>>>(x.sc, q.lv, qb, early);
       }); });
     } else if (shadow) {
       as_const_count(fl.count_work, [&](auto count) { as_const(fl.cull, [&](auto cull) { as_const(fl.wide_shadow, [&](auto wide) {
         if constexpr (count != 1 || !(cull || wide))
           k_query_shadow<count, CRT_REFILL_SHADOW, cull, wide>
-              <<<x->blocks_query_shadow, CRT_TRAV_BLOCK, wide ? dyn_smem(x, CRT_TRAV_BLOCK) : 0, s>>>(x->sc, q.lv, qb, work);
+              <<<x.blocks_query_shadow, CRT_TRAV_BLOCK, wide ? dyn_smem(x, CRT_TRAV_BLOCK) : 0, s>>>(x.sc, q.lv, qb, work);
       }); }); });
     } else {
       as_const(fl.count_work != 0, [&](auto count) { as_const(fl.cull, [&](auto cull) { as_const(fl.wide_closest, [&](auto wide) {
         as_const(primary, [&](auto prim) {
           if constexpr (!(count && wide))
             k_query_closest<prim, count, CRT_REFILL_CLOSEST, cull, wide>
-                <<<x->blocks_query_closest, CRT_TRAV_BLOCK, dyn_smem(x, CRT_TRAV_BLOCK), s>>>(x->sc, q.lv, qb, work);
+                <<<x.blocks_query_closest, CRT_TRAV_BLOCK, dyn_smem(x, CRT_TRAV_BLOCK), s>>>(x.sc, q.lv, qb, work);
         }); }); }); });
     }
   });
@@ -1628,36 +1676,35 @@ static int enqueue_query(crtb200_ctx *x, const Flavour &fl, uint32_t ray_type, c
 
 // The query scratch of GPU x, allocated on first use: work cursors | hand-off counters (ctl, the layout of a frame's
 // queue set), hand-off records for every lane of a query grid up to k_coop's capacity (ovf, all "not published"),
-// device counters, the early pass's side stream, and the span events of the first GPU.
-static int query_scratch(crtb200_ctx *x) {
-  crtb200_ctx::QueueSet &q = x->query;
-  if (x->query_ready) return CRTB200_OK;
+// device counters and the early pass's side stream.
+static int query_scratch(Gpu &x) {
+  QueueSet &q = x.query;
+  if (x.query_ready) return CRTB200_OK;
   int occ = 0;
   CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_query_closest<true, false, CRT_REFILL_CLOSEST, true, false>, CRT_TRAV_BLOCK, 0));
-  x->blocks_query_closest = std::max(1, occ) * x->sm_count;
+  x.blocks_query_closest = std::max(1, occ) * x.sm_count;
   CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_query_shadow<0, CRT_REFILL_SHADOW, true, false>, CRT_TRAV_BLOCK, 0));
-  x->blocks_query_shadow = std::max(1, occ) * x->sm_count;
-  const uint64_t lanes = (uint64_t)std::max(x->blocks_query_closest, x->blocks_query_shadow) * CRT_TRAV_BLOCK;
-  const uint64_t cap = std::min<uint64_t>(lanes, (uint64_t)x->tail_cap * x->blocks_coop * CRT_COOP_WARPS);
+  x.blocks_query_shadow = std::max(1, occ) * x.sm_count;
+  const uint64_t lanes = (uint64_t)std::max(x.blocks_query_closest, x.blocks_query_shadow) * CRT_TRAV_BLOCK;
+  const uint64_t cap = std::min<uint64_t>(lanes, (uint64_t)x.tail_cap * x.blocks_coop * CRT_COOP_WARPS);
   CUDA_TRY(q.ovf.ensure(3 * cap));
   CUDA_TRY(cudaMemset(q.ovf.p, 0xFF, 3 * cap * sizeof(uint4)));
   CUDA_TRY(cudaStreamSynchronize(nullptr));  // (the query runs on the caller's stream, which may not wait for stream 0)
   const size_t n_work = CRT_CTL_STRIDE * (CRT_MAX_LEVELS + 2), n_ovf = CRT_CTL_STRIDE * (CRT_MAX_LEVELS + 1);
   CUDA_TRY(q.ctl.ensure(n_work + n_ovf));
-  CUDA_TRY(x->query_stats_dev.ensure(CRT_STAT_SLOTS));
+  CUDA_TRY(x.query_stats_dev.ensure(CRT_STAT_SLOTS));
   int lo = 0, hi = 0;
   CUDA_TRY(cudaDeviceGetStreamPriorityRange(&lo, &hi));
   // (each part is created once: a call that failed half-way is completed by the next one)
   CUDA_TRY(q.coop_stream.create(cudaStreamNonBlocking, lo));
   CUDA_TRY(q.coop_fork.create(cudaEventDisableTiming));
   CUDA_TRY(q.coop_join.create(cudaEventDisableTiming));
-  for (Event &e : x->query_ev) CUDA_TRY(e.create(cudaEventDefault));
   q.work = q.ctl.p;
   q.lv.ovf = q.ovf.p;
   q.lv.ovf_ctl = q.ctl.p + n_work;
   q.lv.ovf_cap = (uint32_t)cap;
-  q.lv.stats = x->query_stats_dev.p;
-  x->query_ready = true;
+  q.lv.stats = x.query_stats_dev.p;
+  x.query_ready = true;
   return CRTB200_OK;
 }
 
@@ -1670,7 +1717,7 @@ struct HostOut {
 };
 
 // A step of a progressive session (DESIGN.md 3.10.1): global samples [s0, s0 + n) through the chunk loop of
-// enqueue_frame, into the accumulator of the context it runs on.  ap: the stop rule of an adaptive session (DESIGN.md
+// enqueue_frame, into the accumulator of the GPU it runs on.  ap: the stop rule of an adaptive session (DESIGN.md
 // 3.10.2), whose passes compact the active pixels before each sample and run k_adapt_step; null for a plain session.
 struct AccumPass {
   uint32_t s0, n;
@@ -1679,9 +1726,11 @@ struct AccumPass {
 
 // What a frame renders and where its pixels go; callers set the fields they use.
 struct FrameReq {
-  FrameReq(const crtb200_camera *cam, const crtb200_options *o) : cam(cam), o(o) {}
+  FrameReq(const crtb200_camera *cam, const crtb200_options *o, const crtb200_sampling &sampling)
+      : cam(cam), o(o), sampling(sampling) {}
   const crtb200_camera *cam;
   const crtb200_options *o;
+  crtb200_sampling sampling;  // use_gi = 0: unsampled; frame_index is the frame's Philox key word
   float *d_rgb = nullptr;  // device destinations (any may be null)
   uint8_t *d_rgb8 = nullptr;
   HitRec *d_hits = nullptr;
@@ -1692,74 +1741,74 @@ struct FrameReq {
 };
 
 // level-0 work items of tile shard `index` of `count`: 8x4-pixel tiles dealt round-robin, 32 items each
-static uint32_t shard_item_count(const crtb200_ctx *c, uint32_t index, uint32_t count) {
-  const uint32_t tiles = ((c->sc.width + 7) / 8) * ((c->sc.height + 3) / 4);
+static uint32_t shard_item_count(const Gpu &g, uint32_t index, uint32_t count) {
+  const uint32_t tiles = ((g.sc.width + 7) / 8) * ((g.sc.height + 3) / 4);
   return (tiles > index ? (tiles - index + count - 1) / count : 0) * 32u;
 }
 
 // a Frame over the 8x4-pixel tiles of tile shard `index` of `count`, with the mask of the last plan_mask
-static Frame frame_tiles(const crtb200_ctx *c, uint32_t index, uint32_t count) {
+static Frame frame_tiles(const Gpu &g, uint32_t index, uint32_t count) {
   Frame fr{};
-  fr.tiles_x = (c->sc.width + 7) / 8;
-  fr.n_tiles = fr.tiles_x * ((c->sc.height + 3) / 4);
+  fr.tiles_x = (g.sc.width + 7) / 8;
+  fr.n_tiles = fr.tiles_x * ((g.sc.height + 3) / 4);
   fr.shard_index = index;
   fr.shard_count = count;
-  fr.mask = c->mask_needed ? c->mask.p : nullptr;
+  fr.mask = g.mask_needed ? g.mask.p : nullptr;
   return fr;
 }
 
 // One sample pass of one chunk (sample fr.sample): the level loop, the shadow pass, k_accumulate, k_resolve and the
 // kernel that ends a sample of a GI frame or a progressive step
-static int sample_pass(crtb200_ctx *c, const FrameReq &r, const Flavour &fl, Frame &fr, crtb200_ctx::QueueSet &q, uint32_t levels,
-                       bool per_kernel, uint32_t &launches) {
+static int sample_pass(Gpu &g, const FrameReq &r, const Flavour &fl, Frame &fr, QueueSet &q, uint32_t levels,
+                       crtb200_ctx *timed, uint32_t &launches) {
   const cudaStream_t qs = q.stream;
-  const int grid_simple = c->sm_count * 8;
+  const int grid_simple = g.sm_count * 8;
   const bool adapt_step = r.acc && r.acc->ap;
   CUDA_TRY(cudaMemsetAsync(q.ctl.p, 0, q.ctl.n * sizeof(uint32_t), qs));
   if (adapt_step) {
     // level 0 of this pass runs over the pixels still sampling; the host keeps n_items0 as the bound
     fr.list = fr.n_list = nullptr;
     CUDA_TRY(cudaMemsetAsync(q.acount.p, 0, sizeof(uint32_t), qs));
-    k_adapt_compact<<<grid_simple, 256, 0, qs>>>(fr, c->acc_sumsq.p, q.alist.p, q.acount.p);
+    k_adapt_compact<<<grid_simple, 256, 0, qs>>>(fr, g.acc_sumsq.p, q.alist.p, q.acount.p);
     launches++;
     fr.list = q.alist.p;
     fr.n_list = q.acount.p;
   }
-  q.lv.tail_iters = fl.handoff ? (uint32_t)(c->tail_iters + 1) : 0u;
+  q.lv.tail_iters = fl.handoff ? (uint32_t)(g.tail_iters + 1) : 0u;
   q.lv.skip_zero_terms = (r.o->traversal == 0 && r.o->count_work != 1) ? 1u : 0u;
-  q.lv.tail_start = (uint32_t)c->tail_start;
-  q.lv.tail_start_closest = (uint32_t)c->tail_start_closest;
-  q.lv.tail_small = (uint32_t)c->tail_small;
+  q.lv.tail_start = (uint32_t)g.tail_start;
+  q.lv.tail_start_closest = (uint32_t)g.tail_start_closest;
+  q.lv.tail_small = (uint32_t)g.tail_small;
   for (uint32_t l = 0; l < levels; l++) {
-    const int rc = traverse_frame(c, fl, fr, q, false, l, per_kernel, launches);
+    const int rc = traverse_frame(g, fl, fr, q, false, l, timed, launches);
     if (rc) return rc;
-    as_const(fl.gi, [&](auto gi) { k_shade<gi><<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, l); });
+    as_const(fl.gi, [&](auto gi) { k_shade<gi><<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, l); });
     launches += 2;
   }
-  const int rc = traverse_frame(c, fl, fr, q, true, 0, per_kernel, launches);
+  const int rc = traverse_frame(g, fl, fr, q, true, 0, timed, launches);
   if (rc) return rc;
-  k_accumulate<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv);
+  k_accumulate<<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv);
   launches += 2;
   // (GI frames resolve the last level too: its diffuse hits combine D with G background children)
   for (uint32_t l = fl.gi ? levels : levels - 1; l-- > 0;) {
-    as_const(fl.gi, [&](auto gi) { k_resolve<gi><<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, l); });
+    as_const(fl.gi, [&](auto gi) { k_resolve<gi><<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, l); });
     launches++;
   }
   if (adapt_step)
-    k_adapt_step<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, *r.acc->ap, c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p);
+    k_adapt_step<<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, *r.acc->ap, g.acc_sum.p, g.acc_sumsq.p, g.acc_hit.p);
   else if (r.acc)
-    k_accum_step<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, c->acc_sum.p, c->acc_sumsq.p, c->acc_hit.p);
+    k_accum_step<<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, g.acc_sum.p, g.acc_sumsq.p, g.acc_hit.p);
   else if (fl.gi)
-    k_sample_acc<<<grid_simple, 256, 0, qs>>>(c->sc, fr, q.lv, q.acc.p, q.hit0.p);
+    k_sample_acc<<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, q.acc.p, q.hit0.p);
   if (r.acc || fl.gi) launches++;
   return CRTB200_OK;
 }
 
 // the band of image rows that chunk `chunk` (level-0 items [begin, begin + n)) has stored, to the host destinations:
 // behind the chunk's stream qs, on the band stream when there is one
-static int copy_band(crtb200_ctx *c, const FrameReq &r, cudaStream_t qs, uint32_t chunk, uint32_t begin, uint32_t n,
+static int copy_band(crtb200_ctx *c, const Gpu &g, const FrameReq &r, cudaStream_t qs, uint32_t chunk, uint32_t begin, uint32_t n,
                      uint32_t row_items, bool band_stream) {
-  const uint32_t W = c->sc.width, H = c->sc.height;
+  const uint32_t W = g.sc.width, H = g.sc.height;
   const uint32_t row0 = (begin / row_items) * 4u;
   const uint32_t row1 = std::min<uint32_t>(H, ((begin + n + row_items - 1) / row_items) * 4u);
   const size_t off = (size_t)row0 * W, cnt = (size_t)(row1 - row0) * W;
@@ -1784,96 +1833,98 @@ static int copy_band(crtb200_ctx *c, const FrameReq &r, cudaStream_t qs, uint32_
   return CRTB200_OK;
 }
 
-// Enqueue one frame on `st`; c->bands_copied then says whether the frame's host destinations are copied already.
-static int enqueue_frame(crtb200_ctx *c, const FrameReq &r, cudaStream_t st) {
+// Enqueue GPU g's part of one frame on `st`; c->bands_copied then says whether the frame's host destinations are copied
+// already.  Only the context's first GPU records the frame's span and per-launch events: nothing reads another GPU's.
+static int enqueue_frame(crtb200_ctx *c, Gpu &g, const FrameReq &r, cudaStream_t st) {
+  const bool first = &g == c->gpus[0].get();
   const crtb200_options *o = r.o;
   const AccumPass *acc = r.acc;
-  if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
+  if (!g.have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
   if (o->max_depth > 31) return fail(CRTB200_ERR_ARG, "max_depth > 31 is not supported");
   if (o->n_rects && !o->rects) return fail(CRTB200_ERR_ARG, "n_rects > 0 but rects is null");
   if (o->traversal > 1) return fail(CRTB200_ERR_ARG, "unknown traversal mode");
   if (o->count_work > 2) return fail(CRTB200_ERR_ARG, "unknown count_work mode");
-  const Flavour fl = frame_flavour(c, o);
+  const Flavour fl = frame_flavour(g, o, r.sampling);
   const uint32_t shard_count = o->shard_count ? o->shard_count : 1;
   if (o->shard_index >= shard_count) return fail(CRTB200_ERR_ARG, "shard_index >= shard_count");
-  int rc = plan_mask(c, o);
+  int rc = plan_mask(g, o);
   if (rc) return rc;
-  Frame fr = frame_tiles(c, o->shard_index, shard_count);
+  Frame fr = frame_tiles(g, o->shard_index, shard_count);
   for (int k = 0; k < 3; k++) fr.cam.pos[k] = r.cam->position[k];
   for (int k = 0; k < 9; k++) fr.cam.rot[k] = r.cam->rotation[k];
   fr.max_depth = o->max_depth;
   // GI frames (sampling contract, DESIGN.md 3.10): spp sample-major passes per chunk, each the whole level loop
-  const bool gi = fl.gi, secondary = c->has_reflective || c->has_refractive || gi;
+  const bool gi = fl.gi, secondary = g.has_reflective || g.has_refractive || gi;
   fr.resolve = secondary ? 1u : 0u;
   fr.shadow_bias = o->shadow_bias;
   fr.reflection_bias = o->reflection_bias;
   fr.refraction_bias = o->refraction_bias;
   fr.gi = gi ? 1u : 0u;
-  fr.gi_samples = gi ? c->sampling.gi_samples : 0u;
-  fr.spp = gi ? c->sampling.rays_per_pixel : 1u;
-  fr.seed = c->sampling.seed;
-  fr.frame_index = c->sampling.frame_index + c->frame_offset;
-  fr.mc_bias = c->sampling.monte_carlo_bias;
-  const uint32_t shard_items = shard_item_count(c, o->shard_index, shard_count);
+  fr.gi_samples = gi ? r.sampling.gi_samples : 0u;
+  fr.spp = gi ? r.sampling.rays_per_pixel : 1u;
+  fr.seed = r.sampling.seed;
+  fr.frame_index = r.sampling.frame_index;
+  fr.mc_bias = r.sampling.monte_carlo_bias;
+  const uint32_t shard_items = shard_item_count(g, o->shard_index, shard_count);
   // unsharded frames: chunks are whole rows of tiles, so a chunk owns a contiguous band of image rows
   const uint32_t row_items = (shard_count == 1) ? fr.tiles_x * 32u : 32u;
-  rc = plan_queues(c, std::max(shard_items, 32u), o->max_depth, row_items, r.host != nullptr);
+  rc = plan_queues(c, g, r.sampling, std::max(shard_items, 32u), o->max_depth, row_items, r.host != nullptr);
   if (rc) return rc;
   const uint32_t levels = secondary ? o->max_depth + 1 : 1;
-  c->last_samples = acc ? acc->n : fr.spp;
   const uint32_t s_begin = acc ? acc->s0 : 0u, s_end = acc ? acc->s0 + acc->n : fr.spp;
   // Band copies need chunks that own whole rows of tiles: with a small queue budget or a deep refractive scene a chunk
   // is smaller than a tile row, two chunks on different streams would then share a 4-row band and a band copy could
   // pick up the other chunk's stale pixels.  Then the caller copies the whole frame after the join instead.
-  const bool band_copies = r.host && shard_count == 1 && c->cap_items % row_items == 0;
-  c->bands_copied = band_copies;
+  const bool band_copies = r.host && shard_count == 1 && g.cap_items % row_items == 0;
 
   // frames after the first of a batch (crtb200_render_frames) keep accumulating into the same counters and time span
-  if (!r.batch_continuation) CUDA_TRY(cudaMemsetAsync(c->stats_dev.p, 0, CRT_STAT_SLOTS * sizeof(unsigned long long), st));
+  if (!r.batch_continuation) CUDA_TRY(cudaMemsetAsync(g.stats_dev.p, 0, CRT_STAT_SLOTS * sizeof(unsigned long long), st));
 #if CRT_PHASE_CLOCKS
-  CUDA_TRY(cudaMemsetAsync(c->stats_dev.p + CRT_STAT_WARP_SPAN + 3, 0xFF, sizeof(unsigned long long), st));  // atomicMin slots
-  CUDA_TRY(cudaMemsetAsync(c->stats_dev.p + CRT_STAT_WARP_SPAN + 7, 0xFF, sizeof(unsigned long long), st));
+  CUDA_TRY(cudaMemsetAsync(g.stats_dev.p + CRT_STAT_WARP_SPAN + 3, 0xFF, sizeof(unsigned long long), st));  // atomicMin slots
+  CUDA_TRY(cudaMemsetAsync(g.stats_dev.p + CRT_STAT_WARP_SPAN + 7, 0xFF, sizeof(unsigned long long), st));
 #endif
-  c->kev_used = 0;
-  c->kev_kind.clear();
-  if (!r.batch_continuation) CUDA_TRY(cudaEventRecord(c->ev[0], st));
+  if (first) {
+    c->kev_used = 0;
+    c->kev_kind.clear();
+    if (!r.batch_continuation) CUDA_TRY(cudaEventRecord(c->ev[0], st));
+  }
   // fork: every set's stream waits for the caller's stream, chunks go round-robin, the caller's stream joins at the end
-  const uint32_t n_sets = c->cap_sets;
-  const bool per_kernel = n_sets == 1 && !r.batch_continuation;
-  CUDA_TRY(cudaEventRecord(c->fork_ev, st));
-  for (uint32_t k = 0; k < n_sets; k++) CUDA_TRY(cudaStreamWaitEvent(c->sets[k].stream, c->fork_ev, 0));
+  const uint32_t n_sets = g.cap_sets;
+  crtb200_ctx *const timed = first && n_sets == 1 && !r.batch_continuation ? c : nullptr;
+  CUDA_TRY(cudaEventRecord(g.fork_ev, st));
+  for (uint32_t k = 0; k < n_sets; k++) CUDA_TRY(cudaStreamWaitEvent(g.sets[k].stream, g.fork_ev, 0));
   uint32_t launches = 0, chunk = 0;
   // band copies leave on their own stream, so a set starts its next chunk while its last band is still in flight
   const bool band_stream = band_copies && n_sets > 1 && !getenv("CRT_NO_BAND_STREAM");
   if (band_stream) {
     CUDA_TRY(c->band_stream.create(cudaStreamNonBlocking));
     CUDA_TRY(c->band_done.create(cudaEventDisableTiming));
-    if (c->chunk_done.size() < c->n_chunks) c->chunk_done.resize(c->n_chunks);
+    if (c->chunk_done.size() < g.n_chunks) c->chunk_done.resize(g.n_chunks);
     for (Event &e : c->chunk_done) CUDA_TRY(e.create(cudaEventDisableTiming));
   }
-  for (uint32_t begin = 0; begin < shard_items; begin += c->cap_items, chunk++) {
-    crtb200_ctx::QueueSet &q = c->sets[chunk % n_sets];
+  for (uint32_t begin = 0; begin < shard_items; begin += g.cap_items, chunk++) {
+    QueueSet &q = g.sets[chunk % n_sets];
     fr.item_begin = begin;
-    fr.n_items0 = std::min(c->cap_items, shard_items - begin);
+    fr.n_items0 = std::min(g.cap_items, shard_items - begin);
     if (gi && !acc) {
-      CUDA_TRY(q.acc.ensure(c->cap_items));
-      CUDA_TRY(q.hit0.ensure(c->cap_items));
+      CUDA_TRY(q.acc.ensure(g.cap_items));
+      CUDA_TRY(q.hit0.ensure(g.cap_items));
     }
     if (acc && acc->ap) {
-      CUDA_TRY(q.alist.ensure(c->cap_items));
+      CUDA_TRY(q.alist.ensure(g.cap_items));
       CUDA_TRY(q.acount.ensure(1));
     }
     for (uint32_t s = s_begin; s < s_end; s++) {
       fr.sample = s;
-      rc = sample_pass(c, r, fl, fr, q, levels, per_kernel, launches);
+      rc = sample_pass(g, r, fl, fr, q, levels, timed, launches);
       if (rc) return rc;
     }
     if (!acc) {
-      k_store<<<c->sm_count * 8, 256, 0, q.stream>>>(c->sc, fr, q.lv, r.d_rgb, r.d_rgb8, r.d_hits, r.d_slab);
+      k_store<<<g.sm_count * 8, 256, 0, q.stream>>>(g.sc, fr, q.lv, r.d_rgb, r.d_rgb8, r.d_hits, r.d_slab);
       launches++;
     }
     if (band_copies) {
-      rc = copy_band(c, r, q.stream, chunk, begin, fr.n_items0, row_items, band_stream);
+      rc = copy_band(c, g, r, q.stream, chunk, begin, fr.n_items0, row_items, band_stream);
       if (rc) return rc;
     }
   }
@@ -1882,57 +1933,45 @@ static int enqueue_frame(crtb200_ctx *c, const FrameReq &r, cudaStream_t st) {
     CUDA_TRY(cudaStreamWaitEvent(st, c->band_done, 0));
   }
   for (uint32_t k = 0; k < n_sets; k++) {
-    CUDA_TRY(cudaEventRecord(c->sets[k].done, c->sets[k].stream));
-    CUDA_TRY(cudaStreamWaitEvent(st, c->sets[k].done, 0));
+    CUDA_TRY(cudaEventRecord(g.sets[k].done, g.sets[k].stream));
+    CUDA_TRY(cudaStreamWaitEvent(st, g.sets[k].done, 0));
   }
-  CUDA_TRY(cudaEventRecord(c->ev[1], st));
+  if (first) CUDA_TRY(cudaEventRecord(c->ev[1], st));
   CUDA_TRY(cudaGetLastError());
-  c->last.kernel_launches = launches;
-  c->last.levels = levels;
+  g.launches = launches;
+  if (first) {
+    c->last.levels = levels;
+    c->last_samples = acc ? acc->n : fr.spp;
+    c->bands_copied = band_copies;
+  }
   return CRTB200_OK;
 }
 
 // Multi-GPU frame (crtb200_create_multi): shard i of n goes to GPU i; every GPU stores into the SAME destination
-// buffers (device memory of the primary, peer-mapped on the others), and the caller copies the assembled frame to the
-// host after the join.  The peers start after `st` has reached this point (earlier consumers of the frame on the
-// primary's stream are done) and `st` continues after every peer has stored.
+// buffers (device memory of the first GPU, peer-mapped on the others), and the caller copies the assembled frame to the
+// host after the join.  A tile shard of a multi-process frame runs on the first GPU alone.
 static int enqueue_any(crtb200_ctx *c, const FrameReq &r, cudaStream_t st) {
-  if (c->peers.empty() || r.o->shard_count > 1) return enqueue_frame(c, r, st);
-  const uint32_t n = 1u + (uint32_t)c->peers.size();
-  CUDA_TRY(cudaSetDevice(c->device));
-  CUDA_TRY(cudaEventRecord(c->multi_fork, st));
-  crtb200_options o0 = *r.o;
-  o0.shard_index = 0;
-  o0.shard_count = n;
-  FrameReq r0 = r;
-  r0.o = &o0;
-  r0.host = nullptr;
-  int rc = on_all_devices(
-      c, [&] { return enqueue_frame(c, r0, st); },
-      [&](size_t i, crtb200_ctx *p) {
-        crtb200_options oi = *r.o;
-        oi.shard_index = (uint32_t)i + 1u;
-        oi.shard_count = n;
-        FrameReq ri = r0;
-        ri.o = &oi;
-        CUDA_TRY(cudaSetDevice(p->device));
-        CUDA_TRY(cudaStreamWaitEvent(p->stream, c->multi_fork, 0));
-        int e = enqueue_frame(p, ri, p->stream);
-        if (e) return e;
-        p->last_pending = true;
-        CUDA_TRY(cudaEventRecord(p->multi_done, p->stream));
-        return (int)CRTB200_OK;
-      });
-  CUDA_TRY(cudaSetDevice(c->device));
+  const uint32_t n = (uint32_t)c->gpus.size();
+  c->frame_gpus = r.o->shard_count > 1 ? 1u : n;
+  if (c->frame_gpus == 1) return enqueue_frame(c, *c->gpus[0], r, st);
+  const int rc = fan_out(c, n, st, true, [&](uint32_t i, Gpu &g, cudaStream_t s) {
+    crtb200_options oi = *r.o;
+    oi.shard_index = i;
+    oi.shard_count = n;
+    FrameReq ri = r;
+    ri.o = &oi;
+    ri.host = nullptr;
+    return enqueue_frame(c, g, ri, s);
+  });
   if (rc) return rc;
-  for (crtb200_ctx *p : c->peers) CUDA_TRY(cudaStreamWaitEvent(st, p->multi_done, 0));
   CUDA_TRY(cudaEventRecord(c->ev[1], st));  // the frame ends when the last GPU has stored its shard
   return CRTB200_OK;
 }
 
-static int collect_stats_one(crtb200_ctx *c, bool timed) {
+// The counters in a GPU's CRT_STAT_* slots (stats_dev or query_stats_dev), on the current device
+static int read_counts(const unsigned long long *slots, Counts &out) {
   unsigned long long st[CRT_STAT_SLOTS];
-  CUDA_TRY(cudaMemcpy(st, c->stats_dev.p, sizeof(st), cudaMemcpyDeviceToHost));
+  CUDA_TRY(cudaMemcpy(st, slots, sizeof(st), cudaMemcpyDeviceToHost));
 #if CRT_PHASE_CLOCKS
   for (int k = 0; k < 2; k++) {
     const unsigned long long *p = st + CRT_STAT_PHASE + 8 * k;
@@ -1977,111 +2016,125 @@ static int collect_stats_one(crtb200_ctx *c, bool timed) {
               k ? "k_shadow " : "k_closest", g[1], 1e-3 * (double)g[0] / (double)g[1], 1e-3 * (double)(g[2] - g[3]));
   }
 #endif
-  c->last.rays_primary = st[CRT_STAT_RAYS_PRIMARY];
-  c->last.rays_shadow = st[CRT_STAT_RAYS_SHADOW];
-  c->last.rays_reflection = st[CRT_STAT_RAYS_REFLECTION];
-  c->last.rays_refraction = st[CRT_STAT_RAYS_REFRACTION];
-  c->last.node_tests_closest = st[CRT_STAT_NODES_CLOSEST];
-  c->last.triangle_tests_closest = st[CRT_STAT_TRIS_CLOSEST];
-  c->last.node_tests_shadow = st[CRT_STAT_NODES_SHADOW];
-  c->last.triangle_tests_shadow = st[CRT_STAT_TRIS_SHADOW];
-  c->last.handoff_closest = st[CRT_STAT_HANDOFF_CLOSEST];
-  c->last.handoff_shadow = st[CRT_STAT_HANDOFF_SHADOW];
-  c->last.shadow_rays_zero_term = st[CRT_STAT_ZERO_TERM];
-  c->last_side = SideCounts{st[CRT_STAT_DIFFUSE], st[CRT_STAT_PX_SAMPLES], st[CRT_STAT_STOPPED]};
+  crtb200_stats &x = out.s;
+  x.rays_primary = st[CRT_STAT_RAYS_PRIMARY];
+  x.rays_shadow = st[CRT_STAT_RAYS_SHADOW];
+  x.rays_reflection = st[CRT_STAT_RAYS_REFLECTION];
+  x.rays_refraction = st[CRT_STAT_RAYS_REFRACTION];
+  x.node_tests_closest = st[CRT_STAT_NODES_CLOSEST];
+  x.triangle_tests_closest = st[CRT_STAT_TRIS_CLOSEST];
+  x.node_tests_shadow = st[CRT_STAT_NODES_SHADOW];
+  x.triangle_tests_shadow = st[CRT_STAT_TRIS_SHADOW];
+  x.handoff_closest = st[CRT_STAT_HANDOFF_CLOSEST];
+  x.handoff_shadow = st[CRT_STAT_HANDOFF_SHADOW];
+  x.shadow_rays_zero_term = st[CRT_STAT_ZERO_TERM];
+  out.side = SideCounts{st[CRT_STAT_DIFFUSE], st[CRT_STAT_PX_SAMPLES], st[CRT_STAT_STOPPED]};
 #if CRT_COOP_STATS
   fprintf(stderr, "[coop stats] closest: %llu walks, %llu iterations, %llu box tests, %llu triangle tests | shadow: %llu walks, %llu iterations, %llu box tests, %llu triangle tests\n",
           st[CRT_STAT_HANDOFF_CLOSEST], st[CRT_STAT_COOP_DEBUG], st[CRT_STAT_COOP_DEBUG + 1], st[CRT_STAT_COOP_DEBUG + 2],
           st[CRT_STAT_HANDOFF_SHADOW], st[CRT_STAT_COOP_DEBUG + 3], st[CRT_STAT_COOP_DEBUG + 4], st[CRT_STAT_COOP_DEBUG + 5]);
 #endif
-  if (timed) {
-    float ms = 0.f;
-    CUDA_TRY(cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]));
-    c->last.device_ms = ms;
-    c->last.closest_ms = c->last.shadow_ms = c->last.coop_closest_ms = c->last.coop_shadow_ms = 0.0;
-    for (size_t k = 0; k < c->kev_kind.size() && 2 * k + 1 < c->kev_used; k++) {
-      float kms = 0.f;
-      CUDA_TRY(cudaEventElapsedTime(&kms, c->kev[2 * k], c->kev[2 * k + 1]));
-      // closest_ms / shadow_ms include their k_coop part, which is also reported on its own
-      if (c->kev_kind[k] == 0 || c->kev_kind[k] == 2) c->last.closest_ms += kms;
-      if (c->kev_kind[k] == 1 || c->kev_kind[k] == 3) c->last.shadow_ms += kms;
-      if (c->kev_kind[k] == 2) c->last.coop_closest_ms += kms;
-      if (c->kev_kind[k] == 3) c->last.coop_shadow_ms += kms;
-      if (getenv("CRT_KERNEL_TIMES"))  // tools: one line per traversal launch of the frame, in launch order
-        fprintf(stderr, "[kernel times] %s %.3f ms\n", c->kev_kind[k] == 0 ? "k_closest" : c->kev_kind[k] == 1 ? "k_shadow" : "k_coop", kms);
-    }
-  }
   return CRTB200_OK;
 }
 
-// the counters of one render (not its times) added into running totals
-static void add_counts(crtb200_stats &t, SideCounts &tx, const crtb200_stats &s, const SideCounts &sx) {
-  t.rays_primary += s.rays_primary;
-  t.rays_shadow += s.rays_shadow;
-  t.rays_reflection += s.rays_reflection;
-  t.rays_refraction += s.rays_refraction;
-  t.node_tests_closest += s.node_tests_closest;
-  t.triangle_tests_closest += s.triangle_tests_closest;
-  t.node_tests_shadow += s.node_tests_shadow;
-  t.triangle_tests_shadow += s.triangle_tests_shadow;
-  t.handoff_closest += s.handoff_closest;
-  t.handoff_shadow += s.handoff_shadow;
-  t.shadow_rays_zero_term += s.shadow_rays_zero_term;
-  t.kernel_launches += s.kernel_launches;
-  tx.diffuse += sx.diffuse;
-  tx.px_samples += sx.px_samples;
-  tx.stopped += sx.stopped;
+// a record added into running totals: counters, launches and times summed (a GPU's counters carry no time), levels the
+// deepest
+static void add_counts(Counts &t, const Counts &x) {
+  crtb200_stats &a = t.s;
+  const crtb200_stats &b = x.s;
+  a.rays_primary += b.rays_primary;
+  a.rays_shadow += b.rays_shadow;
+  a.rays_reflection += b.rays_reflection;
+  a.rays_refraction += b.rays_refraction;
+  a.node_tests_closest += b.node_tests_closest;
+  a.triangle_tests_closest += b.triangle_tests_closest;
+  a.node_tests_shadow += b.node_tests_shadow;
+  a.triangle_tests_shadow += b.triangle_tests_shadow;
+  a.handoff_closest += b.handoff_closest;
+  a.handoff_shadow += b.handoff_shadow;
+  a.shadow_rays_zero_term += b.shadow_rays_zero_term;
+  a.kernel_launches += b.kernel_launches;
+  a.device_ms += b.device_ms;
+  a.closest_ms += b.closest_ms;
+  a.shadow_ms += b.shadow_ms;
+  a.coop_closest_ms += b.coop_closest_ms;
+  a.coop_shadow_ms += b.coop_shadow_ms;
+  a.levels = std::max(a.levels, b.levels);
+  t.side.diffuse += x.side.diffuse;
+  t.side.px_samples += x.side.px_samples;
+  t.side.stopped += x.side.stopped;
 }
 
-// counters of the primary plus those of the peers (rays, tests, launches); times are the primary's (fork to join)
+// The last render's statistics into c->last / c->last_side: counters and launches summed over the GPUs that rendered
+// it, times of the first GPU (span fork to join, per-launch events)
 static int collect_stats(crtb200_ctx *c) {
-  int rc = collect_stats_one(c, true);
-  if (rc) return rc;
-  for (crtb200_ctx *p : c->peers) {
-    if (!p->last_pending) continue;
-    CUDA_TRY(cudaSetDevice(p->device));
-    CUDA_TRY(cudaStreamSynchronize(p->stream));
-    rc = collect_stats_one(p, false);
-    p->last_pending = false;
+  Counts t;
+  for (uint32_t i = 0; i < c->frame_gpus; i++) {
+    Gpu &g = *c->gpus[i];
+    CUDA_TRY(cudaSetDevice(g.device));
+    if (i) CUDA_TRY(cudaStreamSynchronize(g.stream));
+    Counts x;
+    const int rc = read_counts(g.stats_dev.p, x);
     if (rc) return rc;
-    add_counts(c->last, c->last_side, p->last, p->last_side);
+    x.s.kernel_launches = g.launches;
+    add_counts(t, x);
   }
-  CUDA_TRY(cudaSetDevice(c->device));
+  CUDA_TRY(cudaSetDevice(c->gpus[0]->device));
+  t.s.levels = c->last.levels;
+  float ms = 0.f;
+  CUDA_TRY(cudaEventElapsedTime(&ms, c->ev[0], c->ev[1]));
+  t.s.device_ms = ms;
+  for (size_t k = 0; k < c->kev_kind.size() && 2 * k + 1 < c->kev_used; k++) {
+    float kms = 0.f;
+    CUDA_TRY(cudaEventElapsedTime(&kms, c->kev[2 * k], c->kev[2 * k + 1]));
+    // closest_ms / shadow_ms include their k_coop part, which is also reported on its own
+    if (c->kev_kind[k] == 0 || c->kev_kind[k] == 2) t.s.closest_ms += kms;
+    if (c->kev_kind[k] == 1 || c->kev_kind[k] == 3) t.s.shadow_ms += kms;
+    if (c->kev_kind[k] == 2) t.s.coop_closest_ms += kms;
+    if (c->kev_kind[k] == 3) t.s.coop_shadow_ms += kms;
+    if (getenv("CRT_KERNEL_TIMES"))  // tools: one line per traversal launch of the frame, in launch order
+      fprintf(stderr, "[kernel times] %s %.3f ms\n", c->kev_kind[k] == 0 ? "k_closest" : c->kev_kind[k] == 1 ? "k_shadow" : "k_coop", kms);
+  }
+  c->last = t.s;
+  c->last_side = t.side;
   return CRTB200_OK;
 }
 
 extern "C" {
 
-int crtb200_render(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_options *o, float *rgb_out,
-                   uint8_t *rgb8_out, crtb200_hit *hits_out, crtb200_stats *stats) {
-  ErrScope scope(c);
-  if (!c || !cam || !o) return fail(CRTB200_ERR_ARG, "null argument");
+}  // extern "C"
+
+// crtb200_render of frame `frame` of a batch: the sampling's Philox key word is frame_index + frame
+static int render(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_options *o, uint32_t frame, float *rgb_out,
+                  uint8_t *rgb8_out, crtb200_hit *hits_out, crtb200_stats *stats) {
+  Gpu &g = *c->gpus[0];
   const auto t0 = std::chrono::steady_clock::now();
-  CUDA_TRY(cudaSetDevice(c->device));
-  if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
-  const size_t px = (size_t)c->sc.width * c->sc.height;
+  CUDA_TRY(cudaSetDevice(g.device));
+  if (!g.have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
+  const size_t px = (size_t)g.sc.width * g.sc.height;
   if (hits_out) CUDA_TRY(c->hits.ensure(px));
-  if (hits_out) CUDA_TRY(cudaMemsetAsync(c->hits.p, 0xFF, px * sizeof(HitRec), c->stream));
+  if (hits_out) CUDA_TRY(cudaMemsetAsync(c->hits.p, 0xFF, px * sizeof(HitRec), g.stream));
   c->last = crtb200_stats{};
   // Rectangle grids that leave pixels uncovered keep the previous frame there (colorBuffer persistence), so the whole
   // persistent frame is copied after the render; otherwise each chunk's band is copied as soon as it is stored.
   const HostOut host{rgb_out, rgb8_out, hits_out};
-  int rc = plan_mask(c, o);
+  int rc = plan_mask(g, o);
   if (rc) return rc;
-  FrameReq r(cam, o);
+  FrameReq r(cam, o, c->sampling);
+  r.sampling.frame_index += frame;
   r.d_rgb = c->frame.p;
   r.d_rgb8 = rgb8_out ? c->frame8.p : nullptr;
   r.d_hits = hits_out ? c->hits.p : nullptr;
-  if (o->shard_count <= 1 && !c->mask_needed && (rgb_out || rgb8_out || hits_out)) r.host = &host;
-  rc = enqueue_any(c, r, c->stream);
+  if (o->shard_count <= 1 && !g.mask_needed && (rgb_out || rgb8_out || hits_out)) r.host = &host;
+  rc = enqueue_any(c, r, g.stream);
   if (rc) return rc;
   if (!c->bands_copied) {
-    if (rgb_out) CUDA_TRY(cudaMemcpyAsync(rgb_out, c->frame.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    if (rgb8_out) CUDA_TRY(cudaMemcpyAsync(rgb8_out, c->frame8.p, px * 3, cudaMemcpyDeviceToHost, c->stream));
-    if (hits_out) CUDA_TRY(cudaMemcpyAsync(hits_out, c->hits.p, px * sizeof(HitRec), cudaMemcpyDeviceToHost, c->stream));
+    if (rgb_out) CUDA_TRY(cudaMemcpyAsync(rgb_out, c->frame.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, g.stream));
+    if (rgb8_out) CUDA_TRY(cudaMemcpyAsync(rgb8_out, c->frame8.p, px * 3, cudaMemcpyDeviceToHost, g.stream));
+    if (hits_out) CUDA_TRY(cudaMemcpyAsync(hits_out, c->hits.p, px * sizeof(HitRec), cudaMemcpyDeviceToHost, g.stream));
   }
   const double enqueue_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  CUDA_TRY(cudaStreamSynchronize(g.stream));
   const double sync_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
   rc = collect_stats(c);
   if (rc) return rc;
@@ -2093,7 +2146,7 @@ int crtb200_render(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_opti
       float a = 0.f, b = 0.f;
       cudaEventElapsedTime(&a, c->ev[0], c->dbg_ev[2 * k]);
       cudaEventElapsedTime(&b, c->ev[0], c->dbg_ev[2 * k + 1]);
-      fprintf(stderr, "[chunk times]   chunk %u (up to %u items, set %u): stored at %.3f ms, band on the host at %.3f ms\n", k, c->cap_items, k % c->cap_sets, a, b);
+      fprintf(stderr, "[chunk times]   chunk %u (up to %u items, set %u): stored at %.3f ms, band on the host at %.3f ms\n", k, g.cap_items, k % g.cap_sets, a, b);
     }
     c->dbg_chunks = 0;
   }
@@ -2101,50 +2154,43 @@ int crtb200_render(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_opti
   return CRTB200_OK;
 }
 
-static void add_stats(crtb200_stats &total, SideCounts &tx, const crtb200_stats &s, const SideCounts &sx) {
-  add_counts(total, tx, s, sx);
-  total.device_ms += s.device_ms;
-  total.closest_ms += s.closest_ms;
-  total.shadow_ms += s.shadow_ms;
-  total.coop_closest_ms += s.coop_closest_ms;
-  total.coop_shadow_ms += s.coop_shadow_ms;
-  total.levels = s.levels;
-}
+extern "C" {
 
-// GI frames of a batch: frame f takes Philox key word frame_index + f (on every GPU of a multi-GPU context)
-static void set_frame_offset(crtb200_ctx *c, uint32_t f) {
-  c->frame_offset = f;
-  for (crtb200_ctx *p : c->peers) p->frame_offset = f;
+int crtb200_render(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_options *o, float *rgb_out,
+                   uint8_t *rgb8_out, crtb200_hit *hits_out, crtb200_stats *stats) {
+  ErrScope scope(c);
+  if (!c || !cam || !o) return fail(CRTB200_ERR_ARG, "null argument");
+  return render(c, cam, o, 0, rgb_out, rgb8_out, hits_out, stats);
 }
 
 // The animation loop of app/animation.cpp:24-38 (setCamera + render per frame), batched and pipelined: no host
 // synchronisation between frames, two frames in flight -- frame f + 1 is rendered while frame f's pixels travel to the
 // host on a copy stream.  Rectangle lists that leave pixels uncovered need colorBuffer persistence from frame to frame
-// (one buffer, in order), and tile shards write no full frame: those take the frame-by-frame path.
+// (one buffer, in order), and tile shards write no full frame: those take the frame-by-frame path.  GI frames: frame f
+// takes Philox key word frame_index + f.
 int crtb200_render_frames(crtb200_ctx *c, const crtb200_camera *cams, uint32_t n_frames, const crtb200_options *o,
                           float *rgb_out, uint8_t *rgb8_out, crtb200_stats *stats) {
   ErrScope scope(c);
   if (!c || !cams || !o) return fail(CRTB200_ERR_ARG, "null argument");
-  if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
-  CUDA_TRY(cudaSetDevice(c->device));
-  const size_t px = (size_t)c->sc.width * c->sc.height;
+  Gpu &g = *c->gpus[0];
+  if (!g.have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
+  CUDA_TRY(cudaSetDevice(g.device));
+  const size_t px = (size_t)g.sc.width * g.sc.height;
   const auto t0 = std::chrono::steady_clock::now();
-  int rc = plan_mask(c, o);
+  int rc = plan_mask(g, o);
   if (rc) return rc;
-  if (c->mask_needed || o->shard_count > 1 || o->count_work != 0 || n_frames < 2) {
-    crtb200_stats total{};
-    SideCounts side;
+  if (g.mask_needed || o->shard_count > 1 || o->count_work != 0 || n_frames < 2) {
+    Counts total;
     for (uint32_t f = 0; f < n_frames; f++) {
-      crtb200_stats s{};
-      set_frame_offset(c, f);
-      rc = crtb200_render(c, cams + f, o, rgb_out ? rgb_out + f * px * 3 : nullptr, rgb8_out ? rgb8_out + f * px * 3 : nullptr, nullptr, &s);
-      set_frame_offset(c, 0);
+      Counts x;
+      rc = render(c, cams + f, o, f, rgb_out ? rgb_out + f * px * 3 : nullptr, rgb8_out ? rgb8_out + f * px * 3 : nullptr, nullptr, &x.s);
       if (rc) return rc;
-      add_stats(total, side, s, c->last_side);
+      x.side = c->last_side;
+      add_counts(total, x);
     }
-    total.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    c->last_side = side;
-    if (stats) *stats = total;
+    total.s.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    c->last_side = total.side;
+    if (stats) *stats = total.s;
     return CRTB200_OK;
   }
   CUDA_TRY(c->frame_b.ensure(px * 3));
@@ -2160,23 +2206,22 @@ int crtb200_render_frames(crtb200_ctx *c, const crtb200_camera *cams, uint32_t n
     const int k = (int)(f & 1u);
     float *d_rgb = k ? c->frame_b.p : c->frame.p;
     uint8_t *d_rgb8 = rgb8_out ? (k ? c->frame8_b.p : c->frame8.p) : nullptr;
-    if (f >= 2) CUDA_TRY(cudaStreamWaitEvent(c->stream, c->copied[k], 0));  // this pair's previous frame has left the device
-    set_frame_offset(c, f);
-    FrameReq r(cams + f, o);
+    if (f >= 2) CUDA_TRY(cudaStreamWaitEvent(g.stream, c->copied[k], 0));  // this pair's previous frame has left the device
+    FrameReq r(cams + f, o, c->sampling);
+    r.sampling.frame_index += f;
     r.d_rgb = d_rgb;
     r.d_rgb8 = d_rgb8;
     r.batch_continuation = f > 0;
-    rc = enqueue_any(c, r, c->stream);
-    set_frame_offset(c, 0);
+    rc = enqueue_any(c, r, g.stream);
     if (rc) return rc;
-    launches += c->last.kernel_launches;
-    CUDA_TRY(cudaEventRecord(c->rendered[k], c->stream));
+    launches += g.launches;
+    CUDA_TRY(cudaEventRecord(c->rendered[k], g.stream));
     CUDA_TRY(cudaStreamWaitEvent(c->copy_stream, c->rendered[k], 0));
     if (rgb_out) CUDA_TRY(cudaMemcpyAsync(rgb_out + f * px * 3, d_rgb, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->copy_stream));
     if (rgb8_out) CUDA_TRY(cudaMemcpyAsync(rgb8_out + f * px * 3, d_rgb8, px * 3, cudaMemcpyDeviceToHost, c->copy_stream));
     CUDA_TRY(cudaEventRecord(c->copied[k], c->copy_stream));
   }
-  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  CUDA_TRY(cudaStreamSynchronize(g.stream));
   CUDA_TRY(cudaStreamSynchronize(c->copy_stream));
   if ((n_frames & 1u) == 0u) {  // the last frame went into the second pair: it is the persistent colour buffer now
     std::swap(c->frame, c->frame_b);
@@ -2194,11 +2239,11 @@ int crtb200_render_device(crtb200_ctx *c, const crtb200_camera *cam, const crtb2
                           uint8_t *d_rgb8_out, void *stream) {
   ErrScope scope(c);
   if (!c || !cam || !o) return fail(CRTB200_ERR_ARG, "null argument");
-  CUDA_TRY(cudaSetDevice(c->device));
+  CUDA_TRY(cudaSetDevice(c->gpus[0]->device));
   const uint32_t shard_count = o->shard_count ? o->shard_count : 1;
   c->last = crtb200_stats{};
   c->last_pending = true;
-  FrameReq r(cam, o);
+  FrameReq r(cam, o, c->sampling);
   if (shard_count > 1 && !o->shard_full_frame) {
     // sharded: d_rgb_out is the shard's compact slab (crtb200_shard_items x 3 floats), see crtb200_assemble_shards
     if (d_rgb8_out) return fail(CRTB200_ERR_ARG, "sharded rendering writes a float slab only");
@@ -2213,30 +2258,21 @@ int crtb200_render_device(crtb200_ctx *c, const crtb200_camera *cam, const crtb2
 // ---- progressive sessions (DESIGN.md 3.10.1) ---------------------------------------------------------------------
 // One kernel over the whole tile shard of every GPU of the context: Frame with item_begin 0 and the session's rects;
 // launch(x, fr, stream) enqueues GPU x's kernel.  Queues, device counters, the last render's statistics and the
-// context's sampling stay as they are.  As in enqueue_any, the peers start after c->stream has reached this point and
-// c->stream continues after every peer's kernel.
-static int shard_pass(crtb200_ctx *c, const std::function<void(crtb200_ctx *, const Frame &, cudaStream_t)> &launch) {
-  const std::vector<crtb200_ctx *> gpus = all_gpus(c);
-  const uint32_t n = (uint32_t)gpus.size();
-  if (n > 1) CUDA_TRY(cudaEventRecord(c->multi_fork, c->stream));
-  for (uint32_t i = 0; i < n; i++) {
-    crtb200_ctx *x = gpus[i];
-    CUDA_TRY(cudaSetDevice(x->device));
+// context's sampling stay as they are.  The pass runs on the first GPU's stream (fan_out).
+static int shard_pass(crtb200_ctx *c, const std::function<void(Gpu &, const Frame &, cudaStream_t)> &launch) {
+  const uint32_t n = (uint32_t)c->gpus.size();
+  return fan_out(c, n, c->gpus[0]->stream, false, [&](uint32_t i, Gpu &x, cudaStream_t st) {
     const int rc = plan_mask(x, &c->acc_opt);
     if (rc) return rc;
     Frame fr = frame_tiles(x, i, n);
     fr.n_items0 = shard_item_count(x, i, n);
-    if (i) CUDA_TRY(cudaStreamWaitEvent(x->stream, c->multi_fork, 0));
-    launch(x, fr, x->stream);
+    launch(x, fr, st);
     CUDA_TRY(cudaGetLastError());
-    if (i) CUDA_TRY(cudaEventRecord(x->multi_done, x->stream));
-  }
-  CUDA_TRY(cudaSetDevice(c->device));
-  for (crtb200_ctx *p : c->peers) CUDA_TRY(cudaStreamWaitEvent(c->stream, p->multi_done, 0));
-  return CRTB200_OK;
+    return (int)CRTB200_OK;
+  });
 }
 
-// device staging of a save / load: frame-layout S, Q, hit records and counts on the primary
+// device staging of a save / load: frame-layout S, Q, hit records and counts on the first GPU
 struct AccumStaging {
   DevBuf<float> sum, sumsq;
   DevBuf<HitRec> hit;
@@ -2246,22 +2282,23 @@ struct AccumStaging {
 
 // k_accum_load on every GPU from the staged arrays (all empty: an adaptive begin's flags), then the totals the session
 // keeps on the host.  Inputs that do not fit the scene or `passes` end the session.
-static int accum_load_pass(crtb200_ctx *c, AccumStaging &g, uint32_t passes) {
-  CUDA_TRY(g.bad.ensure(2));
-  CUDA_TRY(g.tot.ensure(3));
-  CUDA_TRY(cudaMemsetAsync(g.bad.p, 0, 2 * sizeof(uint32_t), c->stream));
-  CUDA_TRY(cudaMemsetAsync(g.tot.p, 0, 3 * sizeof(unsigned long long), c->stream));
-  const int rc = shard_pass(c, [&](crtb200_ctx *x, const Frame &fr, cudaStream_t st) {
-    k_accum_load<<<x->sm_count * 8, 256, 0, st>>>(x->sc, fr, g.sum.p, g.sumsq.p, g.hit.p, g.counts.p, passes, x->n_triangles,
-                                                  c->acc_adaptive, c->acc_ap, x->acc_sum.p, x->acc_sumsq.p, x->acc_hit.p,
-                                                  g.bad.p, g.tot.p);
+static int accum_load_pass(crtb200_ctx *c, AccumStaging &stg, uint32_t passes) {
+  Gpu &g = *c->gpus[0];
+  CUDA_TRY(stg.bad.ensure(2));
+  CUDA_TRY(stg.tot.ensure(3));
+  CUDA_TRY(cudaMemsetAsync(stg.bad.p, 0, 2 * sizeof(uint32_t), g.stream));
+  CUDA_TRY(cudaMemsetAsync(stg.tot.p, 0, 3 * sizeof(unsigned long long), g.stream));
+  const int rc = shard_pass(c, [&](Gpu &x, const Frame &fr, cudaStream_t st) {
+    k_accum_load<<<x.sm_count * 8, 256, 0, st>>>(x.sc, fr, stg.sum.p, stg.sumsq.p, stg.hit.p, stg.counts.p, passes, x.n_triangles,
+                                                  c->acc_adaptive, c->acc_ap, x.acc_sum.p, x.acc_sumsq.p, x.acc_hit.p,
+                                                  stg.bad.p, stg.tot.p);
   });
   if (rc) return rc;
   uint32_t bad[2];
   unsigned long long tot[3];
-  CUDA_TRY(cudaMemcpyAsync(bad, g.bad.p, sizeof(bad), cudaMemcpyDeviceToHost, c->stream));
-  CUDA_TRY(cudaMemcpyAsync(tot, g.tot.p, sizeof(tot), cudaMemcpyDeviceToHost, c->stream));
-  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  CUDA_TRY(cudaMemcpyAsync(bad, stg.bad.p, sizeof(bad), cudaMemcpyDeviceToHost, g.stream));
+  CUDA_TRY(cudaMemcpyAsync(tot, stg.tot.p, sizeof(tot), cudaMemcpyDeviceToHost, g.stream));
+  CUDA_TRY(cudaStreamSynchronize(g.stream));
   if (bad[0] || bad[1]) {
     accum_release(c);
     return fail(CRTB200_ERR_ARG, bad[0] ? "hit records name triangles the uploaded scene does not have; the session has ended"
@@ -2277,8 +2314,9 @@ static int accum_load_pass(crtb200_ctx *c, AccumStaging &g, uint32_t passes) {
 static int accum_begin(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_options *o, const crtb200_sampling *s,
                        const crtb200_adaptive *ad) {
   if (!c || !cam || !o || !s) return fail(CRTB200_ERR_ARG, "null argument");
-  CUDA_TRY(cudaSetDevice(c->device));
-  if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
+  Gpu &g = *c->gpus[0];
+  CUDA_TRY(cudaSetDevice(g.device));
+  if (!g.have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
   if (!s->use_gi) return fail(CRTB200_ERR_ARG, "a progressive session needs sampling.use_gi = 1");
   if (ad && ad->min_samples < 2) return fail(CRTB200_ERR_ARG, "adaptive: min_samples must be at least 2");
   if (ad && ad->max_samples < ad->min_samples) return fail(CRTB200_ERR_ARG, "adaptive: max_samples < min_samples");
@@ -2297,38 +2335,37 @@ static int accum_begin(crtb200_ctx *c, const crtb200_camera *cam, const crtb200_
   c->acc_smp = *s;
   c->acc_smp.use_gi = 1;
   c->acc_smp.rays_per_pixel = 1;  // unused: a step says how many samples it renders
-  const std::vector<crtb200_ctx *> gpus = all_gpus(c);
-  const uint32_t n = (uint32_t)gpus.size();
+  const uint32_t n = (uint32_t)c->gpus.size();
   for (uint32_t i = 0; i < n; i++) {
-    crtb200_ctx *x = gpus[i];
-    const size_t items = std::max<size_t>(1, shard_item_count(c, i, n));
-    cudaError_t e = cudaSetDevice(x->device);
-    if (e == cudaSuccess) e = x->acc_sum.ensure(items);
-    if (e == cudaSuccess) e = x->acc_sumsq.ensure(items);
-    if (e == cudaSuccess) e = x->acc_hit.ensure(items);
-    if (e == cudaSuccess) e = cudaMemsetAsync(x->acc_sum.p, 0, items * sizeof(float4), x->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(x->acc_sumsq.p, 0, items * sizeof(float4), x->stream);
+    Gpu &x = *c->gpus[i];
+    const size_t items = std::max<size_t>(1, shard_item_count(g, i, n));
+    cudaError_t e = cudaSetDevice(x.device);
+    if (e == cudaSuccess) e = x.acc_sum.ensure(items);
+    if (e == cudaSuccess) e = x.acc_sumsq.ensure(items);
+    if (e == cudaSuccess) e = x.acc_hit.ensure(items);
+    if (e == cudaSuccess) e = cudaMemsetAsync(x.acc_sum.p, 0, items * sizeof(float4), x.stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(x.acc_sumsq.p, 0, items * sizeof(float4), x.stream);
     // no hit until sample 0 has run: a save at 0 samples must not look up a triangle
-    if (e == cudaSuccess) e = cudaMemsetAsync(x->acc_hit.p, 0xFF, items * sizeof(uint2), x->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(x.acc_hit.p, 0xFF, items * sizeof(uint2), x.stream);
     if (e != cudaSuccess) {
       cudaGetLastError();
       accum_release(c);
       return fail(e == cudaErrorMemoryAllocation ? CRTB200_ERR_MEMORY : CRTB200_ERR_CUDA,
-                  std::string("progressive accumulator (40 bytes per pixel) on device ") + std::to_string(x->device) + ": " +
+                  std::string("progressive accumulator (40 bytes per pixel) on device ") + std::to_string(x.device) + ": " +
                       cudaGetErrorString(e));
     }
   }
-  CUDA_TRY(cudaSetDevice(c->device));
+  CUDA_TRY(cudaSetDevice(g.device));
   c->acc_active = true;
   std::vector<uint8_t> m;
-  c->acc_covered = c->acc_rects.empty() ? (uint64_t)c->sc.width * c->sc.height
-                                        : rect_coverage(c->sc.width, c->sc.height, c->acc_rects, m);
+  c->acc_covered = c->acc_rects.empty() ? (uint64_t)g.sc.width * g.sc.height
+                                        : rect_coverage(g.sc.width, g.sc.height, c->acc_rects, m);
   if (!ad) return CRTB200_OK;
   c->acc_adaptive = true;
   c->acc_ap = AdaptParams{ad->min_samples, ad->max_samples, ad->abs_error, ad->rel_error};
   // every covered pixel starts active: the flags are set on the device, shard by shard
-  AccumStaging g;
-  const int rc = accum_load_pass(c, g, 0);
+  AccumStaging flags;
+  const int rc = accum_load_pass(c, flags, 0);
   if (rc) accum_release(c);
   return rc;
 }
@@ -2348,23 +2385,18 @@ int crtb200_accum_begin_adaptive(crtb200_ctx *c, const crtb200_camera *cam, cons
 int crtb200_accum_step(crtb200_ctx *c, uint32_t n_samples, crtb200_stats *stats) {
   ErrScope scope(c);
   if (!c) return fail(CRTB200_ERR_ARG, "ctx is null");
-  CUDA_TRY(cudaSetDevice(c->device));
+  Gpu &g = *c->gpus[0];
+  CUDA_TRY(cudaSetDevice(g.device));
   if (!c->acc_active) return fail(CRTB200_ERR_STATE, "no progressive session (crtb200_accum_begin)");
   if (n_samples == 0 || (uint64_t)c->acc_done + n_samples > 0xFFFFFFFFull) return fail(CRTB200_ERR_ARG, "n_samples must be at least 1");
   const auto t0 = std::chrono::steady_clock::now();
   c->last = crtb200_stats{};
   const AccumPass a{c->acc_done, n_samples, c->acc_adaptive ? &c->acc_ap : nullptr};
-  // The session's sampling stands in for the context's during the step, because queue planning and the Philox key both
-  // read ctx->sampling; frame_offset is 0 outside crtb200_render_frames, so the key is the session's frame_index.
-  const std::vector<crtb200_ctx *> gpus = all_gpus(c);
-  std::vector<crtb200_sampling> saved;
-  for (crtb200_ctx *x : gpus) saved.push_back(std::exchange(x->sampling, c->acc_smp));
-  FrameReq r(&c->acc_cam, &c->acc_opt);
+  FrameReq r(&c->acc_cam, &c->acc_opt, c->acc_smp);
   r.acc = &a;
-  int rc = enqueue_any(c, r, c->stream);
-  for (size_t i = 0; i < gpus.size(); i++) gpus[i]->sampling = saved[i];
+  int rc = enqueue_any(c, r, g.stream);
   if (rc) return rc;
-  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  CUDA_TRY(cudaStreamSynchronize(g.stream));
   rc = collect_stats(c);
   if (rc) return rc;
   c->acc_done += n_samples;
@@ -2380,58 +2412,60 @@ int crtb200_accum_step(crtb200_ctx *c, uint32_t n_samples, crtb200_stats *stats)
 int crtb200_accum_read(crtb200_ctx *c, float *rgb_out, uint8_t *rgb8_out, crtb200_hit *hits_out, uint32_t *samples_done) {
   ErrScope scope(c);
   if (!c) return fail(CRTB200_ERR_ARG, "ctx is null");
-  CUDA_TRY(cudaSetDevice(c->device));
+  Gpu &g = *c->gpus[0];
+  CUDA_TRY(cudaSetDevice(g.device));
   if (!c->acc_active) return fail(CRTB200_ERR_STATE, "no progressive session (crtb200_accum_begin)");
   if (c->acc_done == 0) return fail(CRTB200_ERR_STATE, "the progressive session has no samples yet");
-  const size_t px = (size_t)c->sc.width * c->sc.height;
+  const size_t px = (size_t)g.sc.width * g.sc.height;
   if (hits_out) CUDA_TRY(c->hits.ensure(px));
-  if (hits_out) CUDA_TRY(cudaMemsetAsync(c->hits.p, 0xFF, px * sizeof(HitRec), c->stream));
-  const int rc = shard_pass(c, [&](crtb200_ctx *x, const Frame &fr, cudaStream_t st) {
-    k_accum_read<<<x->sm_count * 8, 256, 0, st>>>(x->sc, fr, x->acc_sum.p, x->acc_hit.p, c->frame.p,
+  if (hits_out) CUDA_TRY(cudaMemsetAsync(c->hits.p, 0xFF, px * sizeof(HitRec), g.stream));
+  const int rc = shard_pass(c, [&](Gpu &x, const Frame &fr, cudaStream_t st) {
+    k_accum_read<<<x.sm_count * 8, 256, 0, st>>>(x.sc, fr, x.acc_sum.p, x.acc_hit.p, c->frame.p,
                                                   rgb8_out ? c->frame8.p : nullptr, hits_out ? c->hits.p : nullptr);
   });
   if (rc) return rc;
-  if (rgb_out) CUDA_TRY(cudaMemcpyAsync(rgb_out, c->frame.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-  if (rgb8_out) CUDA_TRY(cudaMemcpyAsync(rgb8_out, c->frame8.p, px * 3, cudaMemcpyDeviceToHost, c->stream));
-  if (hits_out) CUDA_TRY(cudaMemcpyAsync(hits_out, c->hits.p, px * sizeof(HitRec), cudaMemcpyDeviceToHost, c->stream));
-  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  if (rgb_out) CUDA_TRY(cudaMemcpyAsync(rgb_out, c->frame.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, g.stream));
+  if (rgb8_out) CUDA_TRY(cudaMemcpyAsync(rgb8_out, c->frame8.p, px * 3, cudaMemcpyDeviceToHost, g.stream));
+  if (hits_out) CUDA_TRY(cudaMemcpyAsync(hits_out, c->hits.p, px * sizeof(HitRec), cudaMemcpyDeviceToHost, g.stream));
+  CUDA_TRY(cudaStreamSynchronize(g.stream));
   if (samples_done) *samples_done = c->acc_done;
   return CRTB200_OK;
 }
 
 // k_accum_save on every GPU into the staged arrays (any may be empty)
-static int accum_save_pass(crtb200_ctx *c, AccumStaging &g) {
-  return shard_pass(c, [&](crtb200_ctx *x, const Frame &fr, cudaStream_t st) {
-    k_accum_save<<<x->sm_count * 8, 256, 0, st>>>(x->sc, fr, x->acc_sum.p, x->acc_sumsq.p, x->acc_hit.p, g.sum.p, g.sumsq.p,
-                                                  g.hit.p, g.counts.p);
+static int accum_save_pass(crtb200_ctx *c, AccumStaging &stg) {
+  return shard_pass(c, [&](Gpu &x, const Frame &fr, cudaStream_t st) {
+    k_accum_save<<<x.sm_count * 8, 256, 0, st>>>(x.sc, fr, x.acc_sum.p, x.acc_sumsq.p, x.acc_hit.p, stg.sum.p, stg.sumsq.p,
+                                                  stg.hit.p, stg.counts.p);
   });
 }
 
 int crtb200_accum_save(crtb200_ctx *c, float *sum_out, float *sumsq_out, crtb200_hit *hit0_out, uint32_t *samples_done) {
   ErrScope scope(c);
   if (!c) return fail(CRTB200_ERR_ARG, "ctx is null");
-  CUDA_TRY(cudaSetDevice(c->device));
+  Gpu &g = *c->gpus[0];
+  CUDA_TRY(cudaSetDevice(g.device));
   if (!c->acc_active) return fail(CRTB200_ERR_STATE, "no progressive session (crtb200_accum_begin)");
-  const size_t px = (size_t)c->sc.width * c->sc.height;
-  AccumStaging g;
+  const size_t px = (size_t)g.sc.width * g.sc.height;
+  AccumStaging stg;
   if (sum_out) {
-    CUDA_TRY(g.sum.ensure(px * 3));
-    CUDA_TRY(cudaMemsetAsync(g.sum.p, 0, px * 3 * sizeof(float), c->stream));
+    CUDA_TRY(stg.sum.ensure(px * 3));
+    CUDA_TRY(cudaMemsetAsync(stg.sum.p, 0, px * 3 * sizeof(float), g.stream));
   }
   if (sumsq_out) {
-    CUDA_TRY(g.sumsq.ensure(px * 3));
-    CUDA_TRY(cudaMemsetAsync(g.sumsq.p, 0, px * 3 * sizeof(float), c->stream));
+    CUDA_TRY(stg.sumsq.ensure(px * 3));
+    CUDA_TRY(cudaMemsetAsync(stg.sumsq.p, 0, px * 3 * sizeof(float), g.stream));
   }
   if (hit0_out) {
-    CUDA_TRY(g.hit.ensure(px));
-    CUDA_TRY(cudaMemsetAsync(g.hit.p, 0xFF, px * sizeof(HitRec), c->stream));
+    CUDA_TRY(stg.hit.ensure(px));
+    CUDA_TRY(cudaMemsetAsync(stg.hit.p, 0xFF, px * sizeof(HitRec), g.stream));
   }
-  const int rc = accum_save_pass(c, g);
+  const int rc = accum_save_pass(c, stg);
   if (rc) return rc;
-  if (sum_out) CUDA_TRY(cudaMemcpyAsync(sum_out, g.sum.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-  if (sumsq_out) CUDA_TRY(cudaMemcpyAsync(sumsq_out, g.sumsq.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-  if (hit0_out) CUDA_TRY(cudaMemcpyAsync(hit0_out, g.hit.p, px * sizeof(HitRec), cudaMemcpyDeviceToHost, c->stream));
-  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  if (sum_out) CUDA_TRY(cudaMemcpyAsync(sum_out, stg.sum.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, g.stream));
+  if (sumsq_out) CUDA_TRY(cudaMemcpyAsync(sumsq_out, stg.sumsq.p, px * 3 * sizeof(float), cudaMemcpyDeviceToHost, g.stream));
+  if (hit0_out) CUDA_TRY(cudaMemcpyAsync(hit0_out, stg.hit.p, px * sizeof(HitRec), cudaMemcpyDeviceToHost, g.stream));
+  CUDA_TRY(cudaStreamSynchronize(g.stream));
   if (samples_done) *samples_done = c->acc_done;
   return CRTB200_OK;
 }
@@ -2440,22 +2474,23 @@ int crtb200_accum_save(crtb200_ctx *c, float *sum_out, float *sumsq_out, crtb200
 static int accum_load(crtb200_ctx *c, const float *sum, const float *sumsq, const crtb200_hit *hit0, const uint32_t *counts,
                       uint32_t samples_done) {
   if (!c || !sum || !sumsq || !hit0) return fail(CRTB200_ERR_ARG, "null argument");
-  CUDA_TRY(cudaSetDevice(c->device));
+  Gpu &g = *c->gpus[0];
+  CUDA_TRY(cudaSetDevice(g.device));
   if (!c->acc_active) return fail(CRTB200_ERR_STATE, "no progressive session (crtb200_accum_begin)");
   if (counts && !c->acc_adaptive) return fail(CRTB200_ERR_ARG, "a counts map can only be loaded into an adaptive session");
-  const size_t px = (size_t)c->sc.width * c->sc.height;
-  AccumStaging g;
-  CUDA_TRY(g.sum.ensure(px * 3));
-  CUDA_TRY(g.sumsq.ensure(px * 3));
-  CUDA_TRY(g.hit.ensure(px));
-  CUDA_TRY(cudaMemcpyAsync(g.sum.p, sum, px * 3 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-  CUDA_TRY(cudaMemcpyAsync(g.sumsq.p, sumsq, px * 3 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-  CUDA_TRY(cudaMemcpyAsync(g.hit.p, hit0, px * sizeof(HitRec), cudaMemcpyHostToDevice, c->stream));
+  const size_t px = (size_t)g.sc.width * g.sc.height;
+  AccumStaging stg;
+  CUDA_TRY(stg.sum.ensure(px * 3));
+  CUDA_TRY(stg.sumsq.ensure(px * 3));
+  CUDA_TRY(stg.hit.ensure(px));
+  CUDA_TRY(cudaMemcpyAsync(stg.sum.p, sum, px * 3 * sizeof(float), cudaMemcpyHostToDevice, g.stream));
+  CUDA_TRY(cudaMemcpyAsync(stg.sumsq.p, sumsq, px * 3 * sizeof(float), cudaMemcpyHostToDevice, g.stream));
+  CUDA_TRY(cudaMemcpyAsync(stg.hit.p, hit0, px * sizeof(HitRec), cudaMemcpyHostToDevice, g.stream));
   if (counts) {
-    CUDA_TRY(g.counts.ensure(px));
-    CUDA_TRY(cudaMemcpyAsync(g.counts.p, counts, px * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(stg.counts.ensure(px));
+    CUDA_TRY(cudaMemcpyAsync(stg.counts.p, counts, px * sizeof(uint32_t), cudaMemcpyHostToDevice, g.stream));
   }
-  const int rc = accum_load_pass(c, g, samples_done);
+  const int rc = accum_load_pass(c, stg, samples_done);
   if (rc) return rc;
   c->acc_done = samples_done;
   return CRTB200_OK;
@@ -2487,23 +2522,25 @@ int crtb200_accum_progress(crtb200_ctx *c, crtb200_progress *p) {
 int crtb200_accum_counts(crtb200_ctx *c, uint32_t *counts_out) {
   ErrScope scope(c);
   if (!c || !counts_out) return fail(CRTB200_ERR_ARG, "null argument");
-  CUDA_TRY(cudaSetDevice(c->device));
+  Gpu &g = *c->gpus[0];
+  CUDA_TRY(cudaSetDevice(g.device));
   if (!c->acc_active) return fail(CRTB200_ERR_STATE, "no progressive session (crtb200_accum_begin)");
-  const size_t px = (size_t)c->sc.width * c->sc.height;
-  AccumStaging g;
-  CUDA_TRY(g.counts.ensure(px));
-  CUDA_TRY(cudaMemsetAsync(g.counts.p, 0, px * sizeof(uint32_t), c->stream));
-  const int rc = accum_save_pass(c, g);
+  const size_t px = (size_t)g.sc.width * g.sc.height;
+  AccumStaging stg;
+  CUDA_TRY(stg.counts.ensure(px));
+  CUDA_TRY(cudaMemsetAsync(stg.counts.p, 0, px * sizeof(uint32_t), g.stream));
+  const int rc = accum_save_pass(c, stg);
   if (rc) return rc;
-  CUDA_TRY(cudaMemcpyAsync(counts_out, g.counts.p, px * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
-  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  CUDA_TRY(cudaMemcpyAsync(counts_out, stg.counts.p, px * sizeof(uint32_t), cudaMemcpyDeviceToHost, g.stream));
+  CUDA_TRY(cudaStreamSynchronize(g.stream));
   return CRTB200_OK;
 }
 
 int crtb200_accum_end(crtb200_ctx *c) {
   ErrScope scope(c);
   if (!c) return fail(CRTB200_ERR_ARG, "ctx is null");
-  CUDA_TRY(cudaSetDevice(c->device));
+  Gpu &g = *c->gpus[0];
+  CUDA_TRY(cudaSetDevice(g.device));
   accum_release(c);
   return CRTB200_OK;
 }
@@ -2511,7 +2548,8 @@ int crtb200_accum_end(crtb200_ctx *c) {
 int crtb200_last_stats(crtb200_ctx *c, crtb200_stats *stats) {
   ErrScope scope(c);
   if (!c || !stats) return fail(CRTB200_ERR_ARG, "null argument");
-  CUDA_TRY(cudaSetDevice(c->device));
+  Gpu &g = *c->gpus[0];
+  CUDA_TRY(cudaSetDevice(g.device));
   if (c->last_pending) {
     CUDA_TRY(cudaEventSynchronize(c->ev[1]));
     int rc = collect_stats(c);
@@ -2525,8 +2563,9 @@ int crtb200_last_stats(crtb200_ctx *c, crtb200_stats *stats) {
 int crtb200_shard_items(crtb200_ctx *c, uint32_t shard_count, uint32_t *items) {
   ErrScope scope(c);
   if (!c || !items || shard_count == 0) return fail(CRTB200_ERR_ARG, "bad argument");
-  if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
-  *items = shard_item_count(c, 0, shard_count);  // shard 0 is the largest
+  Gpu &g = *c->gpus[0];
+  if (!g.have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
+  *items = shard_item_count(*c->gpus[0], 0, shard_count);  // shard 0 is the largest
   return CRTB200_OK;
 }
 
@@ -2570,15 +2609,16 @@ int crtb200_assemble_shards(crtb200_ctx *c, const float *d_slabs, uint32_t shard
                             uint8_t *d_rgb8_out, void *stream) {
   ErrScope scope(c);
   if (!c || !d_slabs || shard_count == 0) return fail(CRTB200_ERR_ARG, "bad argument");
-  if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
-  CUDA_TRY(cudaSetDevice(c->device));
+  Gpu &g = *c->gpus[0];
+  if (!g.have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
+  CUDA_TRY(cudaSetDevice(g.device));
   uint32_t items = 0;
   crtb200_shard_items(c, shard_count, &items);
   // rectangle lists that leave pixels uncovered: the assembled frame keeps what d_rgb_out held there (colorBuffer
   // persistence), exactly like the unsharded path -- the mask is the one of the last render's rectangle list.
   // k_assemble sets the shard of each item itself.
-  const Frame fr = frame_tiles(c, 0, shard_count);
-  k_assemble<<<c->sm_count * 8, 256, 0, (cudaStream_t)stream>>>(c->sc, fr, d_slabs, items, shard_count, d_rgb_out, d_rgb8_out);
+  const Frame fr = frame_tiles(g, 0, shard_count);
+  k_assemble<<<g.sm_count * 8, 256, 0, (cudaStream_t)stream>>>(g.sc, fr, d_slabs, items, shard_count, d_rgb_out, d_rgb8_out);
   CUDA_TRY(cudaGetLastError());
   return CRTB200_OK;
 }
@@ -2586,14 +2626,15 @@ int crtb200_assemble_shards(crtb200_ctx *c, const float *d_slabs, uint32_t shard
 int crtb200_generate_rays_device(crtb200_ctx *c, const crtb200_camera *cam, float *d_rays_out, void *stream) {
   ErrScope scope(c);
   if (!c || !cam) return fail(CRTB200_ERR_ARG, "null argument");
-  if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
-  CUDA_TRY(cudaSetDevice(c->device));
-  int rc = check_device_ptr(c, d_rays_out, 4, "d_rays_out");
+  Gpu &g = *c->gpus[0];
+  if (!g.have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
+  CUDA_TRY(cudaSetDevice(g.device));
+  int rc = check_device_ptr(g, d_rays_out, 4, "d_rays_out");
   if (rc) return rc;
   DCamera dc;
   for (int k = 0; k < 3; k++) dc.pos[k] = cam->position[k];
   for (int k = 0; k < 9; k++) dc.rot[k] = cam->rotation[k];
-  k_generate_rays<<<c->sm_count * 8, 256, 0, (cudaStream_t)stream>>>(c->sc, dc, d_rays_out);
+  k_generate_rays<<<g.sm_count * 8, 256, 0, (cudaStream_t)stream>>>(g.sc, dc, d_rays_out);
   CUDA_TRY(cudaGetLastError());
   return CRTB200_OK;
 }
@@ -2601,24 +2642,26 @@ int crtb200_generate_rays_device(crtb200_ctx *c, const crtb200_camera *cam, floa
 int crtb200_generate_rays(crtb200_ctx *c, const crtb200_camera *cam, float *rays_out) {
   ErrScope scope(c);
   if (!c || !cam || !rays_out) return fail(CRTB200_ERR_ARG, "null argument");
-  if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
-  CUDA_TRY(cudaSetDevice(c->device));
-  const size_t n = (size_t)c->sc.width * c->sc.height;
+  Gpu &g = *c->gpus[0];
+  if (!g.have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
+  CUDA_TRY(cudaSetDevice(g.device));
+  const size_t n = (size_t)g.sc.width * g.sc.height;
   if (n == 0) return CRTB200_OK;
   DevBuf<float> d;
   CUDA_TRY(d.ensure(n * 6));
-  const int rc = crtb200_generate_rays_device(c, cam, d.p, c->stream);
+  const int rc = crtb200_generate_rays_device(c, cam, d.p, g.stream);
   if (rc) return rc;
-  CUDA_TRY(cudaMemcpyAsync(rays_out, d.p, n * 6 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  CUDA_TRY(cudaMemcpyAsync(rays_out, d.p, n * 6 * sizeof(float), cudaMemcpyDeviceToHost, g.stream));
+  CUDA_TRY(cudaStreamSynchronize(g.stream));
   return CRTB200_OK;
 }
 
 int crtb200_scene_trees(crtb200_ctx *c, crtb200_trees *t) {
   ErrScope scope(c);
   if (!c || !t) return fail(CRTB200_ERR_ARG, "null argument");
+  Gpu &g = *c->gpus[0];
   if (!c->trees_built) return fail(CRTB200_ERR_STATE, "the context's scene was not uploaded with crtb200_upload_geometry");
-  CUDA_TRY(cudaSetDevice(c->device));
+  CUDA_TRY(cudaSetDevice(g.device));
   const crtb200_trees &k = c->kd_counts;
   t->n_meshes = k.n_meshes;
   t->n_mesh_nodes = k.n_mesh_nodes;
@@ -2631,13 +2674,13 @@ int crtb200_scene_trees(crtb200_ctx *c, crtb200_trees *t) {
   if (t->meshes && k.n_meshes) std::memcpy(t->meshes, c->kd_meshes.data(), k.n_meshes * sizeof(crtb200_mesh));
   cudaError_t e = cudaSuccess;
   auto get = [&](void *dst, const void *src, size_t bytes) {
-    if (dst && bytes && e == cudaSuccess) e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, c->stream);
+    if (dst && bytes && e == cudaSuccess) e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, g.stream);
   };
   get(t->mesh_nodes, c->kd_nodes.p, (size_t)k.n_mesh_nodes * sizeof(crtb200_kdnode));
   get(t->mesh_leaf_refs, c->kd_refs.p, (size_t)k.n_mesh_leaf_refs * 4);
   get(t->top_nodes, c->kd_nodes.p + k.n_mesh_nodes, (size_t)k.n_top_nodes * sizeof(crtb200_kdnode));
-  get(t->top_leaf_refs, c->top_refs.p, (size_t)k.n_top_leaf_refs * 4);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+  get(t->top_leaf_refs, g.top_refs.p, (size_t)k.n_top_leaf_refs * 4);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(g.stream);
   CUDA_TRY(e);
   return CRTB200_OK;
 }
@@ -2645,29 +2688,29 @@ int crtb200_scene_trees(crtb200_ctx *c, crtb200_trees *t) {
 int crtb200_debug_scene_layout(crtb200_ctx *c, int device_index, crtb200_scene_layout *l) {
   ErrScope scope(c);
   if (!c || !l) return fail(CRTB200_ERR_ARG, "null argument");
-  if (device_index < 0 || (size_t)device_index > c->peers.size()) return fail(CRTB200_ERR_ARG, "device_index out of range");
-  crtb200_ctx *x = device_index ? c->peers[device_index - 1] : c;
-  if (!x->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
+  if (device_index < 0 || (size_t)device_index >= c->gpus.size()) return fail(CRTB200_ERR_ARG, "device_index out of range");
+  Gpu &x = *c->gpus[device_index];
+  if (!x.have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
   static_assert(sizeof(DMesh) == 20, "crtb200_scene_layout.meshes holds 5 words per mesh");
-  l->n_nodes = x->n_nodes;
-  l->n_leaf_refs = x->n_leaf_refs;
-  l->n_top_refs = x->n_top_refs;
-  l->n_meshes = x->sc.n_meshes;
-  l->top_begin = x->sc.top_begin;
-  l->top_end = x->sc.top_end;
-  l->nested_ok = x->nested_ok ? 1u : 0u;
+  l->n_nodes = x.n_nodes;
+  l->n_leaf_refs = x.n_leaf_refs;
+  l->n_top_refs = x.n_top_refs;
+  l->n_meshes = x.sc.n_meshes;
+  l->top_begin = x.sc.top_begin;
+  l->top_end = x.sc.top_end;
+  l->nested_ok = x.nested_ok ? 1u : 0u;
   l->reserved = 0;
-  CUDA_TRY(cudaSetDevice(x->device));
+  CUDA_TRY(cudaSetDevice(x.device));
   cudaError_t e = cudaSuccess;
   auto get = [&](void *dst, const void *src, size_t bytes) {
-    if (dst && bytes && e == cudaSuccess) e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, x->stream);
+    if (dst && bytes && e == cudaSuccess) e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, x.stream);
   };
-  get(l->nodes, x->nodes_p, (size_t)x->n_nodes * 32);
-  get(l->leaf_refs, x->leaf_refs_p, (size_t)x->n_leaf_refs * 4);
-  get(l->top_refs, x->top_refs.p, (size_t)x->n_top_refs * 4);
-  get(l->meshes, x->meshes.p, (size_t)x->sc.n_meshes * sizeof(DMesh));
-  if (e == cudaSuccess) e = cudaStreamSynchronize(x->stream);
-  cudaSetDevice(c->device);
+  get(l->nodes, x.nodes_p, (size_t)x.n_nodes * 32);
+  get(l->leaf_refs, x.leaf_refs_p, (size_t)x.n_leaf_refs * 4);
+  get(l->top_refs, x.top_refs.p, (size_t)x.n_top_refs * 4);
+  get(l->meshes, x.meshes.p, (size_t)x.sc.n_meshes * sizeof(DMesh));
+  if (e == cudaSuccess) e = cudaStreamSynchronize(x.stream);
+  cudaSetDevice(c->gpus[0]->device);
   CUDA_TRY(e);
   return CRTB200_OK;
 }
@@ -2676,22 +2719,24 @@ int crtb200_debug_powf5(crtb200_ctx *c, const float *x, uint32_t n, float *out) 
   ErrScope scope(c);
   if (!c || !x || !out) return fail(CRTB200_ERR_ARG, "null argument");
   if (n == 0) return CRTB200_OK;
-  CUDA_TRY(cudaSetDevice(c->device));
+  Gpu &g = *c->gpus[0];
+  CUDA_TRY(cudaSetDevice(g.device));
   DevBuf<float> dx, dy;
   CUDA_TRY(dx.ensure(n));
   CUDA_TRY(dy.ensure(n));
-  CUDA_TRY(cudaMemcpyAsync(dx.p, x, (size_t)n * 4, cudaMemcpyHostToDevice, c->stream));
-  k_powf5<<<c->sm_count * 8, 256, 0, c->stream>>>(dx.p, n, dy.p);
+  CUDA_TRY(cudaMemcpyAsync(dx.p, x, (size_t)n * 4, cudaMemcpyHostToDevice, g.stream));
+  k_powf5<<<g.sm_count * 8, 256, 0, g.stream>>>(dx.p, n, dy.p);
   CUDA_TRY(cudaGetLastError());
-  CUDA_TRY(cudaMemcpyAsync(out, dy.p, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
-  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  CUDA_TRY(cudaMemcpyAsync(out, dy.p, (size_t)n * 4, cudaMemcpyDeviceToHost, g.stream));
+  CUDA_TRY(cudaStreamSynchronize(g.stream));
   return CRTB200_OK;
 }
 
 // the checks of a ray batch that need no pointer attributes (crtb200_trace_rays_device and its host wrapper)
 static int check_batch(crtb200_ctx *c, const crtb200_ray_batch *b) {
   if (!c || !b || !b->rays) return fail(CRTB200_ERR_ARG, "null argument");
-  if (!c->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
+  Gpu &g = *c->gpus[0];
+  if (!g.have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
   if (b->n >= 0x80000000u) return fail(CRTB200_ERR_ARG, "a ray batch holds fewer than 2^31 rays");
   if (b->ray_type > CRTB200_RAY_REFRACTION) return fail(CRTB200_ERR_ARG, "bad ray type (primary, shadow, reflection or refraction)");
   if (b->traversal > 1) return fail(CRTB200_ERR_ARG, "unknown traversal mode");
@@ -2705,46 +2750,36 @@ int crtb200_trace_rays_device(crtb200_ctx *c, const crtb200_ray_batch *b, void *
   ErrScope scope(c);
   int rc = check_batch(c, b);
   if (rc || b->n == 0) return rc;
-  CUDA_TRY(cudaSetDevice(c->device));
+  Gpu &g = *c->gpus[0];
+  CUDA_TRY(cudaSetDevice(g.device));
   const bool shadow = b->ray_type == CRTB200_RAY_SHADOW;
-  if ((rc = check_device_ptr(c, b->rays, 4, "rays"))) return rc;
-  if (shadow && ((rc = check_device_ptr(c, b->max_distance, 4, "max_distance")) || (rc = check_device_ptr(c, b->occluded, 1, "occluded"))))
+  if ((rc = check_device_ptr(g, b->rays, 4, "rays"))) return rc;
+  if (shadow && ((rc = check_device_ptr(g, b->max_distance, 4, "max_distance")) || (rc = check_device_ptr(g, b->occluded, 1, "occluded"))))
     return rc;
-  if (!shadow && (rc = check_device_ptr(c, b->hits, 4, "hits"))) return rc;
+  if (!shadow && (rc = check_device_ptr(g, b->hits, 4, "hits"))) return rc;
   static_assert(sizeof(HitRec) == sizeof(crtb200_hit), "hit records are written in the public layout");
   // contiguous ranges, one per GPU (a batch smaller than the GPU list uses its first n GPUs)
-  const std::vector<crtb200_ctx *> all = all_gpus(c);
-  const uint32_t g = (uint32_t)std::min<size_t>(all.size(), b->n);
-  for (uint32_t i = 0; i < g; i++) {
-    CUDA_TRY(cudaSetDevice(all[i]->device));
-    if ((rc = query_scratch(all[i]))) return rc;
+  const uint32_t n = (uint32_t)std::min<size_t>(c->gpus.size(), b->n);
+  for (uint32_t i = 0; i < n; i++) {
+    CUDA_TRY(cudaSetDevice(c->gpus[i]->device));
+    if ((rc = query_scratch(*c->gpus[i]))) return rc;
   }
-  CUDA_TRY(cudaSetDevice(c->device));
+  CUDA_TRY(cudaSetDevice(g.device));
+  for (Event &e : c->query_ev) CUDA_TRY(e.create(cudaEventDefault));
   const cudaStream_t st = (cudaStream_t)stream;
-  const Flavour fl = query_flavour(c, b);
+  const Flavour fl = query_flavour(g, b);
   c->query_pending = false;
   CUDA_TRY(cudaEventRecord(c->query_ev[0], st));
-  if (g > 1) CUDA_TRY(cudaEventRecord(c->multi_fork, st));
-  uint32_t launches = 0, forked = 0;
-  for (uint32_t i = 0; i < g && rc == CRTB200_OK; i++) {
-    crtb200_ctx *x = all[i];
-    const uint64_t begin = (uint64_t)b->n * i / g, end = (uint64_t)b->n * (i + 1) / g;
+  uint32_t launches = 0;
+  rc = fan_out(c, n, st, false, [&](uint32_t i, Gpu &x, cudaStream_t xs) {
+    const uint64_t begin = (uint64_t)b->n * i / n, end = (uint64_t)b->n * (i + 1) / n;
     const QueryBatch qb{b->rays + 6 * begin, shadow ? b->max_distance + begin : nullptr,
                         shadow ? nullptr : reinterpret_cast<HitRec *>(b->hits + begin), shadow ? b->occluded + begin : nullptr,
                         (uint32_t)(end - begin)};
-    CUDA_TRY(cudaSetDevice(x->device));
-    const cudaStream_t xs = i ? x->stream : st;
-    if (i) {
-      CUDA_TRY(cudaStreamWaitEvent(xs, c->multi_fork, 0));
-      forked = i;
-    }
-    rc = enqueue_query(x, fl, b->ray_type, qb, xs, launches);
-    if (rc == CRTB200_OK && cudaGetLastError() != cudaSuccess) rc = fail(CRTB200_ERR_CUDA, "a query launch failed");
-    // a peer is joined even when its part failed half-way: what it did enqueue writes into the caller's arrays
-    if (i && cudaEventRecord(x->multi_done, xs) != cudaSuccess && rc == CRTB200_OK) rc = fail(CRTB200_ERR_CUDA, "cudaEventRecord failed");
-  }
-  CUDA_TRY(cudaSetDevice(c->device));
-  for (uint32_t i = 1; i <= forked; i++) CUDA_TRY(cudaStreamWaitEvent(st, all[i]->multi_done, 0));
+    int e = enqueue_query(x, fl, b->ray_type, qb, xs, launches);
+    if (e == CRTB200_OK && cudaGetLastError() != cudaSuccess) e = fail(CRTB200_ERR_CUDA, "a query launch failed");
+    return e;
+  });
   if (rc) return rc;
   CUDA_TRY(cudaEventRecord(c->query_ev[1], st));
   c->query_last = crtb200_stats{};
@@ -2752,7 +2787,7 @@ int crtb200_trace_rays_device(crtb200_ctx *c, const crtb200_ray_batch *b, void *
                        &c->query_last.rays_refraction};
   *rays[b->ray_type] = b->n;
   c->query_last.kernel_launches = launches;
-  c->query_gpus = g;
+  c->query_gpus = n;
   c->query_pending = true;
   return CRTB200_OK;
 }
@@ -2760,26 +2795,22 @@ int crtb200_trace_rays_device(crtb200_ctx *c, const crtb200_ray_batch *b, void *
 int crtb200_last_query_stats(crtb200_ctx *c, crtb200_stats *stats) {
   ErrScope scope(c);
   if (!c || !stats) return fail(CRTB200_ERR_ARG, "null argument");
-  CUDA_TRY(cudaSetDevice(c->device));
+  CUDA_TRY(cudaSetDevice(c->gpus[0]->device));
   if (c->query_pending) {
     CUDA_TRY(cudaEventSynchronize(c->query_ev[1]));
     float ms = 0.f;
     CUDA_TRY(cudaEventElapsedTime(&ms, c->query_ev[0], c->query_ev[1]));
-    crtb200_stats &q = c->query_last;
-    q.device_ms = ms;
-    const std::vector<crtb200_ctx *> all = all_gpus(c);
+    Counts t{c->query_last, {}};
+    t.s.device_ms = ms;
     for (uint32_t i = 0; i < c->query_gpus; i++) {
-      unsigned long long st[CRT_STAT_SLOTS];
-      CUDA_TRY(cudaSetDevice(all[i]->device));
-      CUDA_TRY(cudaMemcpy(st, all[i]->query_stats_dev.p, sizeof(st), cudaMemcpyDeviceToHost));
-      q.node_tests_closest += st[CRT_STAT_NODES_CLOSEST];
-      q.triangle_tests_closest += st[CRT_STAT_TRIS_CLOSEST];
-      q.node_tests_shadow += st[CRT_STAT_NODES_SHADOW];
-      q.triangle_tests_shadow += st[CRT_STAT_TRIS_SHADOW];
-      q.handoff_closest += st[CRT_STAT_HANDOFF_CLOSEST];
-      q.handoff_shadow += st[CRT_STAT_HANDOFF_SHADOW];
+      Counts x;
+      CUDA_TRY(cudaSetDevice(c->gpus[i]->device));
+      const int rc = read_counts(c->gpus[i]->query_stats_dev.p, x);
+      if (rc) return rc;
+      add_counts(t, x);
     }
-    CUDA_TRY(cudaSetDevice(c->device));
+    CUDA_TRY(cudaSetDevice(c->gpus[0]->device));
+    c->query_last = t.s;
     c->query_pending = false;
   }
   *stats = c->query_last;
@@ -2792,17 +2823,18 @@ int crtb200_trace_rays(crtb200_ctx *c, const float *rays, uint32_t n, uint32_t r
   crtb200_ray_batch b{n, ray_type, traversal, 0, rays, max_distance, hits_out, occluded_out};
   int rc = check_batch(c, &b);
   if (rc || n == 0) return rc;
-  CUDA_TRY(cudaSetDevice(c->device));
+  Gpu &g = *c->gpus[0];
+  CUDA_TRY(cudaSetDevice(g.device));
   const bool shadow = ray_type == CRTB200_RAY_SHADOW;
   DevBuf<float> d_rays, d_dist;
   DevBuf<crtb200_hit> d_hits;
   DevBuf<uint8_t> d_occ;
   CUDA_TRY(d_rays.ensure((size_t)n * 6));
-  CUDA_TRY(cudaMemcpyAsync(d_rays.p, rays, (size_t)n * 6 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+  CUDA_TRY(cudaMemcpyAsync(d_rays.p, rays, (size_t)n * 6 * sizeof(float), cudaMemcpyHostToDevice, g.stream));
   if (shadow) {
     CUDA_TRY(d_dist.ensure(n));
     CUDA_TRY(d_occ.ensure(n));
-    CUDA_TRY(cudaMemcpyAsync(d_dist.p, max_distance, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(d_dist.p, max_distance, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, g.stream));
   } else {
     CUDA_TRY(d_hits.ensure(n));
   }
@@ -2810,12 +2842,12 @@ int crtb200_trace_rays(crtb200_ctx *c, const float *rays, uint32_t n, uint32_t r
   b.max_distance = d_dist.p;
   b.hits = d_hits.p;
   b.occluded = d_occ.p;
-  if ((rc = crtb200_trace_rays_device(c, &b, c->stream))) return rc;
+  if ((rc = crtb200_trace_rays_device(c, &b, g.stream))) return rc;
   if (shadow)
-    CUDA_TRY(cudaMemcpyAsync(occluded_out, d_occ.p, n, cudaMemcpyDeviceToHost, c->stream));
+    CUDA_TRY(cudaMemcpyAsync(occluded_out, d_occ.p, n, cudaMemcpyDeviceToHost, g.stream));
   else
-    CUDA_TRY(cudaMemcpyAsync(hits_out, d_hits.p, (size_t)n * sizeof(crtb200_hit), cudaMemcpyDeviceToHost, c->stream));
-  CUDA_TRY(cudaStreamSynchronize(c->stream));
+    CUDA_TRY(cudaMemcpyAsync(hits_out, d_hits.p, (size_t)n * sizeof(crtb200_hit), cudaMemcpyDeviceToHost, g.stream));
+  CUDA_TRY(cudaStreamSynchronize(g.stream));
   return CRTB200_OK;
 }
 

@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE ONLY.  Contexts whose tail hand-off to k_coop (DESIGN.md 3.8) is forced or switched off through the
-tuning environment that crtb200_create reads once per GPU (crtb200_create_multi calls it for every GPU of its list, so
-the peers of a multi-GPU context get the same settings)."""
+tuning environment that context creation reads once per GPU (crtb200_create and crtb200_create_multi read it for every
+GPU of their list, so all GPUs of a multi-GPU context get the same settings)."""
 import os
 
 # every walk still running once the queue is dry (a small frame's queue is dry after the first refill) is handed off

@@ -131,11 +131,6 @@ def test_gi_invariance(gpu, loaded, crt):
     gpu.set_queue_budget(64 << 20)  # >= 3 chunks at this depth
     assert same_f32(_render(gpu, crt, sf, flat, cfg)[0], ref).all()
     gpu.set_queue_budget(16 << 30)
-    multi = crt.Context([0, 0, 0])
-    try:
-        assert same_f32(_render(multi, crt, sf, flat, cfg)[0], ref).all()
-    finally:
-        multi.close()
     # tile shards: compact slabs + assemble
     gpu.upload(flat, keepalive=sf)
     gpu.set_sampling(_smp(crt, cfg))
@@ -160,6 +155,23 @@ def test_gi_invariance(gpu, loaded, crt):
     gpu.set_sampling(None)
     assert not same_f32(frames[0], frames[1]).all()
     assert not same_f32(_render(gpu, crt, sf, flat, cfg, seed=12)[0], ref).all()
+    multi = crt.Context([0, 0, 0])
+    try:
+        assert same_f32(_render(multi, crt, sf, flat, cfg)[0], ref).all()
+        # settings changed after creation hold on every GPU of the context
+        multi.set_concurrency(1)
+        multi.set_queue_budget(64 << 20)
+        assert same_f32(_render(multi, crt, sf, flat, cfg)[0], ref).all()
+        multi.set_queue_budget(16 << 30)
+        multi.set_concurrency(2)
+        # pipelined render_frames: every GPU keys frame f with frame_index + f
+        multi.set_sampling(_smp(crt, cfg))
+        mframes, _, _ = multi.render_frames(cams, crt.make_options(max_depth=cfg["depth"]))
+        multi.set_sampling(None)
+        for f in range(3):
+            assert same_f32(mframes[f], frames[f]).all(), f
+    finally:
+        multi.close()
 
 
 def test_sampling_off_is_unchanged(gpu, loaded, crt):
