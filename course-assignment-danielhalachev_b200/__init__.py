@@ -151,6 +151,14 @@ class RayBatch(C.Structure):
                 ("rays", C.c_void_p), ("max_distance", C.c_void_p), ("hits", C.c_void_p), ("occluded", C.c_void_p)]
 
 
+class ShadeBatch(C.Structure):
+    """crtb200_shade_batch: caller-supplied rays to shade, in device memory (crtb200_shade_rays_device)."""
+    _fields_ = [("n", C.c_uint32), ("ray_type", C.c_uint32), ("traversal", C.c_uint32), ("count_work", C.c_uint32),
+                ("max_depth", C.c_uint32), ("shadow_bias", C.c_float), ("reflection_bias", C.c_float),
+                ("refraction_bias", C.c_float), ("sample", C.c_uint32), ("first_index", C.c_uint32),
+                ("rays", C.c_void_p), ("rgb", C.c_void_p), ("hits", C.c_void_p)]
+
+
 class Hits(NamedTuple):
     """Closest hits of Context.trace: mesh, triangle and t are views of `records`, one (..., 3) int32 tensor in the
     crtb200_hit layout; t holds float32 bits (t.view(torch.float32))."""
@@ -240,6 +248,7 @@ def core() -> C.CDLL:
         lib.crtb200_trace_rays_device.argtypes = [C.c_void_p, C.POINTER(RayBatch), C.c_void_p]
         lib.crtb200_generate_rays_device.argtypes = [C.c_void_p, C.POINTER(Camera), C.c_void_p, C.c_void_p]
         lib.crtb200_last_query_stats.argtypes = [C.c_void_p, C.POINTER(Stats)]
+        lib.crtb200_shade_rays_device.argtypes = [C.c_void_p, C.POINTER(ShadeBatch), C.c_void_p]
         lib.crtb200_device_count.argtypes = [C.POINTER(C.c_int)]
         lib.crtb200_debug_powf5.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]
         lib.crtb200_upload_geometry.argtypes = [C.c_void_p, C.POINTER(Scene)]
@@ -704,6 +713,58 @@ class Context:
         if ray_type == RAY_SHADOW:
             return res
         return Hits(res[..., 0], res[..., 1], res[..., 2], res)
+
+    def shade(self, rays, ray_type: int = RAY_PRIMARY, max_depth: int = 5, bias: float = 1e-4, traversal: int = 0,
+              count_work: int = 0, sample: int = 0, first_index: int = 0, want_hits: bool = False, out=None):
+        """Shades a batch of caller-supplied rays on the GPU (crtb200_shade_rays_device), on torch.cuda.current_stream():
+        colour i is RayTracer::shootRay(ray i, 0) bit for bit, with the context's sampling (GI: ray i is sample `sample`
+        of pixel first_index + i).
+
+        rays: float32 CUDA tensor of shape (..., 6) on the context's first device, contiguous in its last dimension
+        (origin xyz, direction xyz; directions of any length).  ray_type RAY_PRIMARY / RAY_REFLECTION / RAY_REFRACTION;
+        bias is the shadow, reflection and refraction bias.  Returns (rgb, hits): rgb a (..., 3) float32 tensor (out=
+        reuses one), hits a Hits as trace() returns it with want_hits, else None.  Asynchronous like any CUDA work on
+        the stream; last_stats() synchronises."""
+        import torch
+        dev = self._first_device()
+
+        def need(t, what, dtype, shape):
+            if not isinstance(t, torch.Tensor):
+                raise CrtError(f"{what} must be a torch tensor")
+            if t.dtype != dtype:
+                raise CrtError(f"{what} must be {dtype}, not {t.dtype}")
+            if t.device != dev:
+                raise CrtError(f"{what} must be on {dev}, not {t.device}")
+            if tuple(t.shape) != tuple(shape):
+                raise CrtError(f"{what} must have shape {tuple(shape)}, not {tuple(t.shape)}")
+
+        if not isinstance(rays, torch.Tensor) or rays.dim() < 1 or rays.shape[-1] != 6:
+            raise CrtError("rays must be a torch tensor of shape (..., 6)")
+        lead = tuple(rays.shape[:-1])
+        need(rays, "rays", torch.float32, lead + (6,))
+        if ray_type not in (RAY_PRIMARY, RAY_REFLECTION, RAY_REFRACTION):
+            raise CrtError(f"ray_type {ray_type} cannot be shaded (primary, reflection or refraction)")
+        if rays.numel() and rays.stride(-1) != 1:
+            raise CrtError("rays must be contiguous in its last dimension")
+        n = rays.numel() // 6
+        if n >= 1 << 31:
+            raise CrtError(f"a ray batch holds fewer than 2^31 rays, not {n}")
+        flat = rays.reshape(-1, 6).contiguous()  # (a copy on the stream only when the leading dimensions are strided)
+        rgb = out if out is not None else torch.empty(lead + (3,), dtype=torch.float32, device=dev)
+        need(rgb, "out", torch.float32, lead + (3,))
+        if not rgb.is_contiguous():
+            raise CrtError("out must be contiguous")
+        hits = torch.empty(lead + (3,), dtype=torch.int32, device=dev) if want_hits else None
+        b = ShadeBatch(n=n, ray_type=ray_type, traversal=traversal, count_work=count_work, max_depth=max_depth,
+                       shadow_bias=bias, reflection_bias=bias, refraction_bias=bias, sample=sample & 0xFFFFFFFF,
+                       first_index=first_index & 0xFFFFFFFF, rays=flat.data_ptr() or None, rgb=rgb.data_ptr() or None,
+                       hits=hits.data_ptr() if hits is not None and n else None)
+        if n:
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            _check_core(core().crtb200_shade_rays_device(self._h, C.byref(b), stream or None))
+        if hits is None:
+            return rgb, None
+        return rgb, Hits(hits[..., 0], hits[..., 1], hits[..., 2], hits)
 
     def query_stats(self) -> dict:
         """Statistics of the last trace() / trace_rays() (crtb200_last_query_stats; waits for the query to finish): rays

@@ -15,6 +15,9 @@
 //   Q   k_query_closest / k_query_shadow / k_coop_query
 //                                   caller-supplied ray batches on the same loop and hand-off (walk kinds
 //                                   QueryClosestWalk / QueryShadowWalk, k_coop's body with the ray source CoopQuerySrc)
+//   S   k_closest_rays / k_coop_rays / k_shade_rays / k_resolve_rays / k_store_rays
+//                                   caller-supplied rays shaded through the frame pipeline: level 0 of a chunk reads the
+//                                   caller's rays (walk kind RaysClosestWalk, sources CoopRaysSrc / RaysLevel0)
 //
 // Reference functions replaced are cited at each kernel.  No tensor cores: the path is pointer-chasing + scalar
 // binary32 arithmetic; the B200-specific choices are the 32-byte-sector node records, L2-resident working set,
@@ -654,10 +657,41 @@ static __device__ __noinline__ void spawn_diffuse(const Frame &fr, const Levels 
   }
 }
 
+// Where level 0 of k_shade / k_resolve comes from (the caller's rays: RaysLevel0, with the shade kernels at the end):
+//   valid(sc, fr, i)                    level-0 slot i holds a ray
+//   ray<GI>(sc, fr, i, valid, o, d, key, pix, n)  valid: slot i holds a ray; then its ray, GI: its root path key and
+//                                                 pixel index, and n += 1
+//   stat()                              the CRT_STAT_RAYS_* slot its rays count in
+// CameraLevel0: the pixel of the tile mapping and its (jittered) camera ray.  (ray() keeps the statement structure
+// k_shade had before the sources existed: the register allocation of k_shade<false> depends on it.)
+struct CameraLevel0 {
+  template <bool GI>
+  CRT_DI bool valid(const DScene &sc, const Frame &fr, const uint32_t i) const {
+    uint32_t row, col;
+    return item_pixel<GI>(fr, sc, fr.item_begin + i, row, col);
+  }
+  template <bool GI>
+  CRT_DI void ray(const DScene &sc, const Frame &fr, const uint32_t i, bool &valid, V3 &o, V3 &d, uint32_t &key,
+                  uint32_t &pix, uint32_t &n) const {
+    uint32_t row, col;
+    valid = item_pixel<GI>(fr, sc, fr.item_begin + i, row, col);
+    if (valid) {
+      if (GI) {
+        key = jittered_primary_ray(fr, sc.width, sc.height, row, col, o, d);
+        pix = row * sc.width + col;
+      } else {
+        primary_ray(fr.cam, sc.width, sc.height, row, col, o, d);
+      }
+      n++;
+    }
+  }
+  CRT_DI uint32_t stat() const { return CRT_STAT_RAYS_PRIMARY; }
+};
+
 // GI: frames under the sampling contract (crt_sampling.h): jittered level 0, path keys carried in ray_o.w / pixel index in
 // ray_d.w, and every diffuse hit also spawns G diffuse children (COMB_GI).  GI = false is the unsampled kernel.
-template <bool GI>
-__global__ void __launch_bounds__(256) k_shade(const DScene sc, const Frame fr, const Levels lv, const uint32_t level) {
+template <bool GI, class L0>
+CRT_DI void shade_level(const DScene &sc, const Frame &fr, const Levels &lv, const uint32_t level, const L0 &src) {
   const uint32_t total = (level == 0) ? level0_items<GI>(fr) : lv.counts[level];
   const uint32_t node_base = lv.offset[level];
   const uint32_t rounded = (total + 31u) & ~31u;
@@ -669,17 +703,7 @@ __global__ void __launch_bounds__(256) k_shade(const DScene sc, const Frame fr, 
     uint32_t key = 0, pix = 0;  // GI: path key of this ray, global pixel index
     if (valid) {
       if (level == 0) {
-        uint32_t row, col;
-        valid = item_pixel<GI>(fr, sc, fr.item_begin + i, row, col);
-        if (valid) {
-          if (GI) {
-            key = jittered_primary_ray(fr, sc.width, sc.height, row, col, o, d);
-            pix = row * sc.width + col;
-          } else {
-            primary_ray(fr.cam, sc.width, sc.height, row, col, o, d);
-          }
-          n_prim++;
-        }
+        src.template ray<GI>(sc, fr, i, valid, o, d, key, pix, n_prim);
       } else {
         const float4 ro = lv.ray_o[node - lv.offset[1]];
         const float4 rd = lv.ray_d[node - lv.offset[1]];
@@ -822,11 +846,16 @@ __global__ void __launch_bounds__(256) k_shade(const DScene sc, const Frame fr, 
       }
     }
   }
-  // ray statistics (traced rays only, SURVEY 8(d))
-  warp_stat_add(lv, CRT_STAT_RAYS_PRIMARY, (unsigned long long)n_prim);
+  // ray statistics (traced rays only, SURVEY 8(d)); n_prim: level-0 rays, counted under the source's type
+  warp_stat_add(lv, src.stat(), (unsigned long long)n_prim);
   warp_stat_add(lv, CRT_STAT_RAYS_REFLECTION, (unsigned long long)n_refl);
   warp_stat_add(lv, CRT_STAT_RAYS_REFRACTION, (unsigned long long)n_refr);
   if (GI) warp_stat_add(lv, CRT_STAT_DIFFUSE, (unsigned long long)n_diff);
+}
+
+template <bool GI>
+__global__ void __launch_bounds__(256) k_shade(const DScene sc, const Frame fr, const Levels lv, const uint32_t level) {
+  shade_level<GI>(sc, fr, lv, level, CameraLevel0{});
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -1383,16 +1412,13 @@ __global__ void __launch_bounds__(256) k_accumulate(const DScene sc, const Frame
 // ------------------------------------------------------------------------------------------------------------
 //   GI diffuse : (D + base (*) S) / float(G + 1), S = ((0 + L_0) + L_1) + ...,   D = the light sum k_accumulate left in
 //                color[node], base from the diffuse item (sampling contract, DESIGN.md 3.10)
-template <bool GI>
-__global__ void __launch_bounds__(256) k_resolve(const DScene sc, const Frame fr, const Levels lv, const uint32_t level) {
+template <bool GI, class L0>
+CRT_DI void resolve_level(const DScene &sc, const Frame &fr, const Levels &lv, const uint32_t level, const L0 &src) {
   const uint32_t total = (level == 0) ? level0_items<GI>(fr) : lv.counts[level];
   const uint32_t node_base = lv.offset[level];
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
     const uint32_t node = node_base + i;
-    if (level == 0) {
-      uint32_t row, col;
-      if (!item_pixel<GI>(fr, sc, fr.item_begin + i, row, col)) continue;
-    }
+    if (level == 0 && !src.template valid<GI>(sc, fr, i)) continue;
     const uint4 cb = lv.comb[node];
     if (cb.x == COMB_FINAL) continue;
     if (GI && cb.x == COMB_GI) {
@@ -1421,6 +1447,11 @@ __global__ void __launch_bounds__(256) k_resolve(const DScene sc, const Frame fr
     }
     lv.color[node] = make_float4(out.x, out.y, out.z, 0.f);
   }
+}
+
+template <bool GI>
+__global__ void __launch_bounds__(256) k_resolve(const DScene sc, const Frame fr, const Levels lv, const uint32_t level) {
+  resolve_level<GI>(sc, fr, lv, level, CameraLevel0{});
 }
 
 // Sample pass fr.sample of a GI frame: acc = acc + c_s in sample order (acc starts at (0,0,0)); the last pass leaves
@@ -1997,6 +2028,141 @@ __global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_co
                                                                                        const uint32_t early) {
   __shared__ WarpCoop s_wc[CRT_COOP_WARPS];
   coop_walks<SHADOW, PRIMARY, true, CRT_COOP_GROUP, true>(sc, lv, 0u, early, s_wc[threadIdx.x >> 5], CoopQuerySrc{qb});
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// Caller-supplied rays shaded through the frame pipeline (crtb200_shade_rays_device, DESIGN.md 3.13): RayTracer::shootRay
+// (RayTracer.cpp:419-451) for a batch of rays.  Level 0 of a chunk is ray item_begin + i of the batch instead of a
+// pixel; every later level, the shadow pass, k_accumulate and the resolve of levels > 0 are the frame's kernels.  Four
+// places derive a level-0 ray, each has a kernel of its own here: the closest-hit walk (k_closest_rays), its hand-off
+// (k_coop_rays), k_shade_rays and k_resolve_rays; k_store_rays writes colour i and hit i.
+// ------------------------------------------------------------------------------------------------------------
+struct ShadeRays {
+  const float *rays;     // this GPU's range of the batch: n x 6 (origin xyz, direction xyz)
+  float *rgb;            // n x 3
+  HitRec *hits;          // n, or null
+  uint32_t first_index;  // GI: pixel index p of ray 0 of the range
+  uint32_t stat;         // CRT_STAT_RAYS_* slot of the batch's ray type
+};
+
+// Ray `item` of the range with shootRay's normalisation of the direction (RayTracer.cpp:420), applied once: the walk,
+// its hand-off and k_shade read the same bits
+CRT_DI void shade_ray(const ShadeRays &sr, const uint32_t item, V3 &o, V3 &d) {
+  Ray r;
+  query_ray(sr.rays, item, r);
+  o = r.o;
+  d = vnorm(r.d);
+}
+
+struct RaysLevel0 {
+  const ShadeRays &sr;
+  template <bool GI>
+  CRT_DI bool valid(const DScene &, const Frame &, const uint32_t) const { return true; }
+  // GI: p = first_index + item, s = fr.sample, root path key = R(p, s, 0, 0).z (the word jittered_primary_ray returns)
+  template <bool GI>
+  CRT_DI void ray(const DScene &, const Frame &fr, const uint32_t i, bool &valid, V3 &o, V3 &d, uint32_t &key,
+                  uint32_t &pix, uint32_t &n) const {
+    shade_ray(sr, fr.item_begin + i, o, d);
+    if (GI) {
+      pix = sr.first_index + fr.item_begin + i;
+      key = crt_s_philox(pix, fr.sample, 0u, 0u, fr.seed, fr.frame_index).z;
+    }
+    valid = true;
+    n++;
+  }
+  CRT_DI uint32_t stat() const { return sr.stat; }
+};
+
+// Level 0's closest-hit walk: ClosestWalk over the chunk's n_items0 rays of the batch.  PRIMARY (CRTB200_RAY_PRIMARY
+// batches): the primary ray's back-face rule, independent of where the ray comes from.
+template <bool P>
+struct RaysClosestWalk : ClosestWalk<P, false> {
+  const uint32_t total;
+  const ShadeRays &sr;
+  CRT_DI RaysClosestWalk(const Frame &fr, const Levels &lv, const ShadeRays &s) : ClosestWalk<P, false>(fr, lv, 0u), total(fr.n_items0), sr(s) {}
+  CRT_DI bool take(const DScene &, const Frame &fr, const Levels &, const uint32_t i, Ray &ray, uint32_t &) const {
+    shade_ray(sr, fr.item_begin + i, ray.o, ray.d);
+    return true;
+  }
+};
+
+template <bool PRIMARY, bool COUNT, int REFILL, bool CULL, bool WIDE>
+__global__ void __launch_bounds__(CRT_TRAV_BLOCK, CRT_TRAV_MIN_BLOCKS) k_closest_rays(const DScene sc, const Frame fr, const Levels lv, const ShadeRays sr,
+                                                                                   uint32_t *__restrict__ work_counter) {
+  __shared__ WarpShare s_ws[CRT_TRAV_BLOCK / 32];
+  WarpShare &ws = s_ws[threadIdx.x >> 5];
+  RaysClosestWalk<PRIMARY> w(fr, lv, sr);
+  walk_loop<REFILL, CULL, WIDE, false, (COUNT ? 0 : (WIDE ? 2 : 1)), COUNT, !COUNT, false>(sc, fr, lv, work_counter, ws, w);
+}
+
+// The ray source of k_coop_rays: record id = level-0 queue node id
+struct CoopRaysSrc {
+  const Frame &fr;
+  const ShadeRays &sr;
+  template <bool SHADOW, bool PRIMARY>
+  CRT_DI void ray(const DScene &, const Levels &lv, const uint32_t id, Ray &ray, float &) const {
+    shade_ray(sr, fr.item_begin + (id - lv.offset[0]), ray.o, ray.d);
+  }
+  CRT_DI float shadow_limit(const Ray &ray, const float dist) const { return crtd::shadow_limit(ray, dist); }
+  CRT_DI void shadow_answer(const Levels &, const uint32_t, const bool) const {}
+  CRT_DI void closest_answer(const DScene &, const Levels &lv, const uint32_t id, const Closest &cl) const {
+    lv.hit_tri[id] = cl.best_tri;
+    lv.hit_t[id] = cl.best_t;
+  }
+};
+
+// k_coop over the level-0 walks k_closest_rays handed off
+template <bool PRIMARY, bool CULL>
+__global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_coop_rays(const DScene sc, const Frame fr, const Levels lv, const ShadeRays sr,
+                                                                                      const uint32_t early) {
+  __shared__ WarpCoop s_wc[CRT_COOP_WARPS];
+  coop_walks<false, PRIMARY, CULL, CRT_COOP_GROUP, true>(sc, lv, 0u, early, s_wc[threadIdx.x >> 5], CoopRaysSrc{fr, sr});
+}
+
+template <bool GI>
+__global__ void __launch_bounds__(256) k_shade_rays(const DScene sc, const Frame fr, const Levels lv, const ShadeRays sr) {
+  shade_level<GI>(sc, fr, lv, 0u, RaysLevel0{sr});
+}
+
+template <bool GI>
+__global__ void __launch_bounds__(256) k_resolve_rays(const DScene sc, const Frame fr, const Levels lv, const ShadeRays sr) {
+  resolve_level<GI>(sc, fr, lv, 0u, RaysLevel0{sr});
+}
+
+// Colour i and hit i of the chunk's rays, in place of k_store: a warp's 32 colours leave as 24 16-byte stores when rgb is
+// 16-byte aligned (chunks start at multiples of 32 rays, so every full warp's 384 bytes are then aligned too).  Counts
+// the chunk's shadow rays as k_store does.
+__global__ void __launch_bounds__(256) k_store_rays(const DScene sc, const Frame fr, const Levels lv, const ShadeRays sr) {
+  __shared__ __align__(16) float s_f[8][96];
+  if (blockIdx.x == 0 && threadIdx.x == 0)
+    atomicAdd(&lv.stats[CRT_STAT_RAYS_SHADOW], (unsigned long long)lv.counts[CRT_MAX_LEVELS] * sc.n_lights);
+  const uint32_t lane = lane_id(), w = threadIdx.x >> 5;
+  const bool aligned = (reinterpret_cast<uintptr_t>(sr.rgb) & 15u) == 0u;
+  for (uint32_t base = blockIdx.x * blockDim.x + (threadIdx.x & ~31u); base < fr.n_items0; base += gridDim.x * blockDim.x) {
+    const uint32_t i = base + lane, k = fr.item_begin + i;
+    const bool valid = i < fr.n_items0;
+    const float4 c = valid ? lv.color[lv.offset[0] + i] : make_float4(0.f, 0.f, 0.f, 0.f);
+    if (aligned && base + 32u <= fr.n_items0) {
+      s_f[w][3 * lane + 0] = c.x;
+      s_f[w][3 * lane + 1] = c.y;
+      s_f[w][3 * lane + 2] = c.z;
+      __syncwarp();
+      if (lane < 24u)
+        *reinterpret_cast<float4 *>(sr.rgb + 3 * (size_t)(fr.item_begin + base) + 4 * lane) = *reinterpret_cast<const float4 *>(&s_f[w][4 * lane]);
+      __syncwarp();
+    } else if (valid) {
+      sr.rgb[3 * (size_t)k + 0] = c.x;
+      sr.rgb[3 * (size_t)k + 1] = c.y;
+      sr.rgb[3 * (size_t)k + 2] = c.z;
+    }
+    if (sr.hits && valid) {
+      const uint32_t tri = lv.hit_tri[lv.offset[0] + i];
+      HitRec h;
+      public_tri(sc, tri, h);
+      h.t = tri == CRT_INVALID ? 0.0f : lv.hit_t[lv.offset[0] + i];
+      sr.hits[k] = h;
+    }
+  }
 }
 
 }  // namespace crtd

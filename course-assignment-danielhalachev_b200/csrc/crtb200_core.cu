@@ -1523,6 +1523,7 @@ static int check_device_ptr(const Gpu &g, const void *p, size_t align, const cha
 struct Flavour {
   uint32_t count_work;
   bool cull, handoff, gi, wide_closest, wide_shadow;
+  const ShadeRays *rays = nullptr;  // level 0 reads this range of a caller's rays (crtb200_shade_rays_device), not pixels
 };
 
 static Flavour frame_flavour(const Gpu &g, const crtb200_options *o, const crtb200_sampling &smp) {
@@ -1552,9 +1553,19 @@ static void as_const_count(uint32_t v, F &&f) {
   v == 1 ? f(std::integral_constant<int, 1>{}) : v == 2 ? f(std::integral_constant<int, 2>{}) : f(std::integral_constant<int, 0>{});
 }
 
-// k_closest of level `level`: PRIMARY at level 0, jittered in GI frames
+// k_closest of level `level`: PRIMARY at level 0, jittered in GI frames; level 0 of caller rays: k_closest_rays, PRIMARY
+// for primary batches
 static void launch_closest(const Gpu &g, const Flavour &fl, const Frame &fr, QueueSet &q, uint32_t level) {
   const bool primary = level == 0;
+  if (fl.rays && primary) {
+    as_const(fl.count_work != 0, [&](auto count) { as_const(fl.cull, [&](auto cull) { as_const(fl.wide_closest, [&](auto wide) {
+      as_const(fl.rays->stat == CRT_STAT_RAYS_PRIMARY, [&](auto prim) {
+        if constexpr (!(count && wide))
+          k_closest_rays<prim, count, CRT_REFILL_CLOSEST, cull, wide>
+              <<<g.blocks_closest, CRT_TRAV_BLOCK, dyn_smem(g, CRT_TRAV_BLOCK), q.stream>>>(g.sc, fr, q.lv, *fl.rays, q.work);
+      }); }); }); });
+    return;
+  }
   as_const(fl.count_work != 0, [&](auto count) { as_const(fl.cull, [&](auto cull) { as_const(fl.wide_closest, [&](auto wide) {
     as_const(primary, [&](auto prim) { as_const(primary && fl.gi, [&](auto jitter) {
       if constexpr (!(count && wide) && (prim || !jitter))
@@ -1576,6 +1587,12 @@ static void launch_shadow(const Gpu &g, const Flavour &fl, const Frame &fr, Queu
 // k_coop over the walks the shadow pass or closest-hit level `level` handed off; SKIPR = false in GI shadow passes
 static void launch_coop(const Gpu &g, const Flavour &fl, const Frame &fr, QueueSet &q, bool shadow, uint32_t level,
                         int blocks, cudaStream_t st, uint32_t early) {
+  if (fl.rays && !shadow && level == 0) {  // (k_coop's PRIMARY source would regenerate camera rays)
+    as_const(fl.rays->stat == CRT_STAT_RAYS_PRIMARY, [&](auto prim) { as_const(fl.cull, [&](auto cull) {
+      k_coop_rays<prim, cull><<<blocks, 32 * CRT_COOP_WARPS, 0, st>>>(g.sc, fr, q.lv, *fl.rays, early);
+    }); });
+    return;
+  }
   as_const(shadow, [&](auto sh) { as_const(!shadow && level == 0, [&](auto prim) { as_const(fl.cull, [&](auto cull) {
     as_const(!(shadow && fl.gi), [&](auto skipr) {
       if constexpr (!(sh && prim) && (sh || skipr))
@@ -1738,6 +1755,10 @@ struct FrameReq {
   const HostOut *host = nullptr;    // crtb200_render: band copies where the frame allows them (ctx->bands_copied)
   bool batch_continuation = false;  // a frame after the first of crtb200_render_frames
   const AccumPass *acc = nullptr;   // a step of a progressive session
+  // crtb200_shade_rays_device: level 0 is this GPU's range of n_rays caller rays (cam is null), one pass with sample word
+  // `sample`; colours and hits go to rays->rgb / rays->hits
+  const ShadeRays *rays = nullptr;
+  uint32_t n_rays = 0, sample = 0;
 };
 
 // level-0 work items of tile shard `index` of `count`: 8x4-pixel tiles dealt round-robin, 32 items each
@@ -1782,7 +1803,12 @@ static int sample_pass(Gpu &g, const FrameReq &r, const Flavour &fl, Frame &fr, 
   for (uint32_t l = 0; l < levels; l++) {
     const int rc = traverse_frame(g, fl, fr, q, false, l, timed, launches);
     if (rc) return rc;
-    as_const(fl.gi, [&](auto gi) { k_shade<gi><<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, l); });
+    as_const(fl.gi, [&](auto gi) {
+      if (fl.rays && l == 0)
+        k_shade_rays<gi><<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, *fl.rays);
+      else
+        k_shade<gi><<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, l);
+    });
     launches += 2;
   }
   const int rc = traverse_frame(g, fl, fr, q, true, 0, timed, launches);
@@ -1791,16 +1817,23 @@ static int sample_pass(Gpu &g, const FrameReq &r, const Flavour &fl, Frame &fr, 
   launches += 2;
   // (GI frames resolve the last level too: its diffuse hits combine D with G background children)
   for (uint32_t l = fl.gi ? levels : levels - 1; l-- > 0;) {
-    as_const(fl.gi, [&](auto gi) { k_resolve<gi><<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, l); });
+    as_const(fl.gi, [&](auto gi) {
+      if (fl.rays && l == 0)
+        k_resolve_rays<gi><<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, *fl.rays);
+      else
+        k_resolve<gi><<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, l);
+    });
     launches++;
   }
+  // (a batch of caller rays is one pass with an arbitrary sample word: nothing to average)
+  const bool sample_acc = fl.gi && !fl.rays;
   if (adapt_step)
     k_adapt_step<<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, *r.acc->ap, g.acc_sum.p, g.acc_sumsq.p, g.acc_hit.p);
   else if (r.acc)
     k_accum_step<<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, g.acc_sum.p, g.acc_sumsq.p, g.acc_hit.p);
-  else if (fl.gi)
+  else if (sample_acc)
     k_sample_acc<<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, q.acc.p, q.hit0.p);
-  if (r.acc || fl.gi) launches++;
+  if (r.acc || sample_acc) launches++;
   return CRTB200_OK;
 }
 
@@ -1844,14 +1877,17 @@ static int enqueue_frame(crtb200_ctx *c, Gpu &g, const FrameReq &r, cudaStream_t
   if (o->n_rects && !o->rects) return fail(CRTB200_ERR_ARG, "n_rects > 0 but rects is null");
   if (o->traversal > 1) return fail(CRTB200_ERR_ARG, "unknown traversal mode");
   if (o->count_work > 2) return fail(CRTB200_ERR_ARG, "unknown count_work mode");
-  const Flavour fl = frame_flavour(g, o, r.sampling);
+  Flavour fl = frame_flavour(g, o, r.sampling);
+  fl.rays = r.rays;
   const uint32_t shard_count = o->shard_count ? o->shard_count : 1;
   if (o->shard_index >= shard_count) return fail(CRTB200_ERR_ARG, "shard_index >= shard_count");
-  int rc = plan_mask(g, o);
+  int rc = r.rays ? CRTB200_OK : plan_mask(g, o);
   if (rc) return rc;
   Frame fr = frame_tiles(g, o->shard_index, shard_count);
-  for (int k = 0; k < 3; k++) fr.cam.pos[k] = r.cam->position[k];
-  for (int k = 0; k < 9; k++) fr.cam.rot[k] = r.cam->rotation[k];
+  if (r.cam) {
+    for (int k = 0; k < 3; k++) fr.cam.pos[k] = r.cam->position[k];
+    for (int k = 0; k < 9; k++) fr.cam.rot[k] = r.cam->rotation[k];
+  }
   fr.max_depth = o->max_depth;
   // GI frames (sampling contract, DESIGN.md 3.10): spp sample-major passes per chunk, each the whole level loop
   const bool gi = fl.gi, secondary = g.has_reflective || g.has_refractive || gi;
@@ -1861,17 +1897,18 @@ static int enqueue_frame(crtb200_ctx *c, Gpu &g, const FrameReq &r, cudaStream_t
   fr.refraction_bias = o->refraction_bias;
   fr.gi = gi ? 1u : 0u;
   fr.gi_samples = gi ? r.sampling.gi_samples : 0u;
-  fr.spp = gi ? r.sampling.rays_per_pixel : 1u;
+  fr.spp = gi && !r.rays ? r.sampling.rays_per_pixel : 1u;
   fr.seed = r.sampling.seed;
   fr.frame_index = r.sampling.frame_index;
   fr.mc_bias = r.sampling.monte_carlo_bias;
-  const uint32_t shard_items = shard_item_count(g, o->shard_index, shard_count);
+  const uint32_t shard_items = r.rays ? r.n_rays : shard_item_count(g, o->shard_index, shard_count);
   // unsharded frames: chunks are whole rows of tiles, so a chunk owns a contiguous band of image rows
-  const uint32_t row_items = (shard_count == 1) ? fr.tiles_x * 32u : 32u;
+  const uint32_t row_items = (shard_count == 1 && !r.rays) ? fr.tiles_x * 32u : 32u;
   rc = plan_queues(c, g, r.sampling, std::max(shard_items, 32u), o->max_depth, row_items, r.host != nullptr);
   if (rc) return rc;
   const uint32_t levels = secondary ? o->max_depth + 1 : 1;
-  const uint32_t s_begin = acc ? acc->s0 : 0u, s_end = acc ? acc->s0 + acc->n : fr.spp;
+  // sample passes s_begin, s_begin + 1, ... (caller rays: one, with any sample word)
+  const uint32_t s_begin = acc ? acc->s0 : (r.rays ? r.sample : 0u), n_passes = acc ? acc->n : fr.spp;
   // Band copies need chunks that own whole rows of tiles: with a small queue budget or a deep refractive scene a chunk
   // is smaller than a tile row, two chunks on different streams would then share a 4-row band and a band copy could
   // pick up the other chunk's stale pixels.  Then the caller copies the whole frame after the join instead.
@@ -1906,7 +1943,7 @@ static int enqueue_frame(crtb200_ctx *c, Gpu &g, const FrameReq &r, cudaStream_t
     QueueSet &q = g.sets[chunk % n_sets];
     fr.item_begin = begin;
     fr.n_items0 = std::min(g.cap_items, shard_items - begin);
-    if (gi && !acc) {
+    if (gi && !acc && !r.rays) {
       CUDA_TRY(q.acc.ensure(g.cap_items));
       CUDA_TRY(q.hit0.ensure(g.cap_items));
     }
@@ -1914,12 +1951,15 @@ static int enqueue_frame(crtb200_ctx *c, Gpu &g, const FrameReq &r, cudaStream_t
       CUDA_TRY(q.alist.ensure(g.cap_items));
       CUDA_TRY(q.acount.ensure(1));
     }
-    for (uint32_t s = s_begin; s < s_end; s++) {
-      fr.sample = s;
+    for (uint32_t k = 0; k < n_passes; k++) {
+      fr.sample = s_begin + k;
       rc = sample_pass(g, r, fl, fr, q, levels, timed, launches);
       if (rc) return rc;
     }
-    if (!acc) {
+    if (r.rays) {
+      k_store_rays<<<g.sm_count * 8, 256, 0, q.stream>>>(g.sc, fr, q.lv, *r.rays);
+      launches++;
+    } else if (!acc) {
       k_store<<<g.sm_count * 8, 256, 0, q.stream>>>(g.sc, fr, q.lv, r.d_rgb, r.d_rgb8, r.d_hits, r.d_slab);
       launches++;
     }
@@ -2848,6 +2888,55 @@ int crtb200_trace_rays(crtb200_ctx *c, const float *rays, uint32_t n, uint32_t r
   else
     CUDA_TRY(cudaMemcpyAsync(hits_out, d_hits.p, (size_t)n * sizeof(crtb200_hit), cudaMemcpyDeviceToHost, g.stream));
   CUDA_TRY(cudaStreamSynchronize(g.stream));
+  return CRTB200_OK;
+}
+
+// Caller rays through the frame pipeline (DESIGN.md 3.13): each GPU's contiguous range is a frame request whose level 0
+// is that range (enqueue_frame's chunk loop, sample_pass's level loop), fanned out as frames are.
+int crtb200_shade_rays_device(crtb200_ctx *c, const crtb200_shade_batch *b, void *stream) {
+  ErrScope scope(c);
+  if (!c || !b || !b->rays || !b->rgb) return fail(CRTB200_ERR_ARG, "null argument");
+  if (b->n >= 0x80000000u) return fail(CRTB200_ERR_ARG, "a ray batch holds fewer than 2^31 rays");
+  if (b->ray_type != CRTB200_RAY_PRIMARY && b->ray_type != CRTB200_RAY_REFLECTION && b->ray_type != CRTB200_RAY_REFRACTION)
+    return fail(CRTB200_ERR_ARG, "bad ray type (primary, reflection or refraction)");
+  if (b->traversal > 1) return fail(CRTB200_ERR_ARG, "unknown traversal mode");
+  if (b->count_work > 2) return fail(CRTB200_ERR_ARG, "unknown count_work mode");
+  if (b->max_depth > 31) return fail(CRTB200_ERR_ARG, "max_depth > 31 is not supported");
+  Gpu &g = *c->gpus[0];
+  if (!g.have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
+  if (b->n == 0) return CRTB200_OK;
+  CUDA_TRY(cudaSetDevice(g.device));
+  int rc;
+  if ((rc = check_device_ptr(g, b->rays, 4, "rays")) || (rc = check_device_ptr(g, b->rgb, 4, "rgb")) ||
+      (b->hits && (rc = check_device_ptr(g, b->hits, 4, "hits"))))
+    return rc;
+  crtb200_options o{};
+  o.max_depth = b->max_depth;
+  o.shadow_bias = b->shadow_bias;
+  o.reflection_bias = b->reflection_bias;
+  o.refraction_bias = b->refraction_bias;
+  o.traversal = b->traversal;
+  o.count_work = b->count_work;
+  const uint32_t stat = b->ray_type == CRTB200_RAY_PRIMARY ? CRT_STAT_RAYS_PRIMARY
+                        : b->ray_type == CRTB200_RAY_REFLECTION ? CRT_STAT_RAYS_REFLECTION : CRT_STAT_RAYS_REFRACTION;
+  const cudaStream_t st = (cudaStream_t)stream;
+  c->last = crtb200_stats{};
+  c->last_pending = true;
+  // contiguous ranges, one per GPU, as crtb200_trace_rays_device splits a batch; a range keeps its global p
+  const uint32_t n = (uint32_t)std::min<size_t>(c->gpus.size(), b->n);
+  c->frame_gpus = n;
+  rc = fan_out(c, n, st, true, [&](uint32_t i, Gpu &x, cudaStream_t xs) {
+    const uint64_t begin = (uint64_t)b->n * i / n, end = (uint64_t)b->n * (i + 1) / n;
+    const ShadeRays sr{b->rays + 6 * begin, b->rgb + 3 * begin, b->hits ? reinterpret_cast<HitRec *>(b->hits + begin) : nullptr,
+                       b->first_index + (uint32_t)begin, stat};
+    FrameReq r(nullptr, &o, c->sampling);
+    r.rays = &sr;
+    r.n_rays = (uint32_t)(end - begin);
+    r.sample = b->sample;
+    return enqueue_frame(c, x, r, xs);
+  });
+  if (rc) return rc;
+  if (n > 1) CUDA_TRY(cudaEventRecord(c->ev[1], st));  // the call ends when the last GPU has stored its range
   return CRTB200_OK;
 }
 

@@ -465,6 +465,42 @@ int crtb200_last_query_stats(crtb200_ctx *ctx, crtb200_stats *stats);
 int crtb200_trace_rays(crtb200_ctx *ctx, const float *rays, uint32_t n, uint32_t ray_type, uint32_t traversal,
                        const float *max_distance, crtb200_hit *hits_out, uint8_t *occluded_out);
 
+/* A batch of caller-supplied rays to shade, in DEVICE memory of the context's first GPU (DESIGN.md 3.13). */
+typedef struct crtb200_shade_batch {
+  uint32_t n;            /* rays; n < 2^31 (CRTB200_ERR_ARG otherwise); 0 = nothing to do                              */
+  uint32_t ray_type;     /* CRTB200_RAY_PRIMARY (the primary ray's back-face rule) / _REFLECTION / _REFRACTION          */
+  uint32_t traversal;    /* as crtb200_options.traversal                                                               */
+  uint32_t count_work;   /* as crtb200_options.count_work                                                              */
+  uint32_t max_depth;    /* MAX_DEPTH, <= 31                                                                           */
+  float shadow_bias, reflection_bias, refraction_bias;
+  uint32_t sample;       /* GI only: Philox counter word s of every ray of the batch                                   */
+  uint32_t first_index;  /* GI only: ray i is "pixel" p = first_index + i (mod 2^32)                                   */
+  const float *rays;     /* n * 6 float32: origin xyz, direction xyz (any length)                                      */
+  float *rgb;            /* n * 3 float32, required                                                                    */
+  crtb200_hit *hits;     /* n records, optional: the ray's own closest hit (public numbering; miss: -1, -1, t = 0)     */
+} crtb200_shade_batch;
+
+/* replaces: RayTracer::shootRay(ray, 0) (RayTracer.cpp:419-451) for a batch of caller-supplied rays: colour i is bit for
+ * bit shootRay of ray i, including its normalisation of the direction (:420), under the batch's ray type, max_depth and
+ * biases.  shootRay(ray, d) under MAX_DEPTH = M is shootRay(ray, 0) under MAX_DEPTH = M - d, so no depth argument
+ * exists.  With the context's sampling on (crtb200_set_sampling) a ray is one GI sample: key {seed, frame_index},
+ * pixel p = first_index + i, sample s = `sample`, root path key R(p, s, 0, 0).z -- the jittered camera ray of pixel p's
+ * sample s shaded this way is that sample of a GI frame; rays_per_pixel is ignored.  Shading the once-normalised getRay
+ * ray of each pixel with sampling off gives crtb200_render's frame.  The answers do not depend on traversal, the tail
+ * hand-off, the queue budget, the GPU list, the stream, or how a GI batch is split into calls (given first_index).
+ * The rays run through the frame pipeline (level loop, shadow pass, resolve).  On a crtb200_create_multi context the
+ * batch is split into contiguous ranges, one per GPU, each writing its colours and hits into the first GPU's memory
+ * through the peer mapping.  Asynchronous on `stream` (a cudaStream_t, NULL = default), with the same rule about
+ * concurrent use of one context as crtb200_render_device.  After synchronisation crtb200_last_stats and
+ * crtb200_last_sampling_stats describe this call: level-0 rays under the batch's type, shadow, secondary and diffuse
+ * rays, tests under count_work, hand-offs, device_ms, kernel_launches.  The colour buffer, a progressive session and
+ * crtb200_last_query_stats are untouched.
+ * CRTB200_ERR_ARG: null batch / rays / rgb; rays, rgb or a non-null hits not device memory of the context's first GPU or
+ * not 4-byte aligned; CRTB200_RAY_SHADOW, _DIFFUSE or an unknown ray type; traversal > 1, count_work > 2,
+ * max_depth > 31, n >= 2^31.  CRTB200_ERR_STATE without a scene.  CRTB200_ERR_MEMORY when the ray tree does not fit
+ * the queue budget, as for frames. */
+int crtb200_shade_rays_device(crtb200_ctx *ctx, const crtb200_shade_batch *batch, void *stream);
+
 /* Test hook: evaluates the device's (1 - cos)^5 routine (csrc/crt_powf5.h), the stand-in for glibc's
  * std::powf(x, 5) of RayTracer.cpp:407, on n host floats -- so the parity suite can check it bit for bit against libm. */
 int crtb200_debug_powf5(crtb200_ctx *ctx, const float *x, uint32_t n, float *out);
