@@ -1,6 +1,6 @@
 // crt_kernels.cuh -- the wavefront pipeline kernels (sm_100a).
 //
-//   K1  primary-ray generation      fused into k_closest<PRIMARY> / k_shade (level 0) + standalone k_generate_rays
+//   K1  primary-ray generation      fused into k_closest<CameraRays> / k_shade (level 0) + standalone k_generate_rays
 //   K2  k_closest                   persistent closest-hit traversal, one ray per lane, stack-free two-level KD walk
 //   K4/K5 k_shade                   per-hit: barycentrics, smooth normal, texture sample, material switch,
 //                                   reflect / refract + Fresnel, compaction of children into the next level's queue
@@ -11,13 +11,11 @@
 //                                   (k_mark tells it that the kernel has ended), a final pass behind both
 //   K3c k_accumulate                in-order light sum per diffuse hit
 //   K6  k_resolve                   bottom-up combine of the ray tree in the reference's expression order
-//   K7  k_store                     level-0 colours -> framebuffer (f32 + PPMColor u8)
-//   Q   k_query_closest / k_query_shadow / k_coop_query
-//                                   caller-supplied ray batches on the same loop and hand-off (walk kinds
-//                                   QueryClosestWalk / QueryShadowWalk, k_coop's body with the ray source CoopQuerySrc)
-//   S   k_closest_rays / k_coop_rays / k_shade_rays / k_resolve_rays / k_store_rays
-//                                   caller-supplied rays shaded through the frame pipeline: level 0 of a chunk reads the
-//                                   caller's rays (walk kind RaysClosestWalk, sources CoopRaysSrc / RaysLevel0)
+//   K7  k_store                     level-0 colours -> framebuffer (f32 + PPMColor u8); k_store_rays for caller rays
+// k_closest, k_shadow, k_coop, k_shade and k_resolve take a ray source as a template and a kernel parameter (see "Ray
+// sources"): a frame's queue (QueueRays), camera rays (CameraRays) and (hit, light) pairs (ShadowPairs), a caller's
+// rays shaded through the frame pipeline (ShadeRays), a caller's closest-hit and shadow queries (QueryClosest /
+// QueryShadow).
 //
 // Reference functions replaced are cited at each kernel.  No tensor cores: the path is pointer-chasing + scalar
 // binary32 arithmetic; the B200-specific choices are the 32-byte-sector node records, L2-resident working set,
@@ -406,8 +404,8 @@ CRT_DI bool tail_handoff(const Levels &lv, const uint32_t launch, const bool wan
 // MODE: 2 = this loop.  (0 = while-while and 1 = merged single loop were the round-1 predecessors; their measurements are
 // in profiles/r1_tuning.md, their code is gone.)
 //
-// A walk kind (ClosestWalk, ShadowWalk) holds the per-lane state of a walk's answer and supplies the steps that differ.
-// `id` is where the answer goes (the ray's queue node / the pair's visibility slot), also the hand-off record's id:
+// A walk kind (ClosestWalk, ShadowWalk, each over a ray source) holds the per-lane state of a walk's answer and supplies
+// the steps that differ.  `id` is the source's record id of the ray, where its answer goes and the hand-off record's id:
 //   total, take(i, ray, id)  work items of the launch; the ray of item i (false: the item is answered without a walk)
 //   begin(ray, i, id)        a new walk's answer state; tri_dist() = w of its entry in the warp's ray table
 //   limit(), allow_behind()  the node phase's culling bound (node_test)
@@ -536,29 +534,67 @@ CRT_DI void walk_loop(const DScene &sc, const Frame &fr, const Levels &lv, uint3
 
 // ------------------------------------------------------------------------------------------------------------
 // K2: closest hit.  Replaces RayTracer::trace -> KDTree<ObjectKDTreeSubTree>::intersect -> KDTree<Triangle>::intersect
-// (RayTracer.cpp:453-458, KDTree.cpp:127-166, 48-87).  Work item = one ray of `level` (level 0: a pixel of the chunk);
-// the answer is the ray node's hit_tri / hit_t.
-// JITTER (PRIMARY only): level 0 of a GI frame, jittered primary rays (a template flag, so that the unsampled primary
-// kernels keep their register allocation)
+// (RayTracer.cpp:453-458, KDTree.cpp:127-166, 48-87).  Work item = one ray of the launch's source; the answer is its
+// closest hit (a frame's: the ray node's hit_tri / hit_t).
+//
+// Ray sources (here the frame's QueueRays and CameraRays; ShadowPairs with K3, ShadeRays and the query sources at the end).
+// A source says where the rays of a launch come from and where their answers go.  k_closest / k_shadow walk its items
+// and k_coop reads the walks they hand off through the same source object, so a walk and its hand-off read the same
+// ray bits.  Per-kernel flags (F: JITTER of k_closest, ZERO_TERMS of k_shadow, GI of k_shade / k_resolve) reach it as
+// member-template arguments; the back-face rule (PRIMARY) is the kernel's own flag.
+//   SHADOW                                   its rays are shadow rays (k_shadow) or closest-hit rays (k_closest)
+//   level(l)                                 the level of a launch at `l`; 0 for the caller's rays, whose launches are
+//                                            level 0 by construction (also the hand-off line of a closest-hit launch)
+//   items<F>(fr, lv, level), base(lv, level) closest hit: work items of the launch, record id of item 0 (id = base + i)
+//   take<F>(sc, fr, lv, base, i, ray)        closest hit: the ray of item i; false: not a ray of the launch
+//   base(lv), items(sc, base)                shadow: a word of the launch take() reads, work items
+//   take<F>(sc, fr, lv, base, i, ray, dist, id, n)  shadow: the ray of item i, its distance bound and record id; false:
+//                                            answered without a walk (n += 1)
+//   ray(sc, fr, lv, id, ray, dist)           the ray of record id again (k_coop); shadow: with its distance bound
+//   limit(ray, dist), declined(lv, n)        shadow: the culling bound (CULL); counts the items take() declined
+//   answer(sc, lv, id, cl) / answer(lv, id, occluded)  where a closest hit / an occlusion answer goes
+// The level-0 sources of a frame request (CameraRays, ShadeRays) also feed level 0 of k_shade / k_resolve:
+//   valid<GI>(sc, fr, i)                     level-0 slot i holds a ray
+//   level0<GI>(sc, fr, i, valid, o, d, key, pix, n)  valid: slot i holds a ray; then its ray, GI: its root path key and
+//                                            pixel index, and n += 1
+//   ray_stat()                               the CRT_STAT_RAYS_* slot its rays count in
 // ------------------------------------------------------------------------------------------------------------
-template <bool P, bool JITTER>
-struct ClosestWalk {
-  static constexpr bool PRIMARY = P, SHADOW = false;
-  static constexpr uint32_t STAT_NODES = CRT_STAT_NODES_CLOSEST, STAT_TRIS = CRT_STAT_TRIS_CLOSEST;
-  const uint32_t level, total, node_base;
-  Closest cl;
-  CRT_DI ClosestWalk(const Frame &fr, const Levels &lv, const uint32_t lvl)
-      : level(lvl), total(PRIMARY ? level0_items<JITTER>(fr) : lv.counts[lvl]), node_base(lv.offset[lvl]) {
-    closest_begin(cl);
+// The frame's rays of level > 0: node base + i of the queue.  Its launches are the frame's secondary levels (k_closest's
+// CRT_TRAV_MIN_BLOCKS_SEC).
+struct QueueRays {
+  static constexpr bool SHADOW = false;
+  CRT_DI uint32_t level(const uint32_t l) const { return l; }
+  template <bool>
+  CRT_DI uint32_t items(const Frame &, const Levels &lv, const uint32_t level) const { return lv.counts[level]; }
+  CRT_DI uint32_t base(const Levels &lv, const uint32_t level) const { return lv.offset[level]; }
+  template <bool>
+  CRT_DI bool take(const DScene &, const Frame &, const Levels &lv, const uint32_t base, const uint32_t i, Ray &ray) const {
+    const float4 o = lv.ray_o[base - lv.offset[1] + i];
+    const float4 d = lv.ray_d[base - lv.offset[1] + i];
+    ray.o = mk(o.x, o.y, o.z);
+    ray.d = mk(d.x, d.y, d.z);
+    return true;
   }
-  CRT_DI bool take(const DScene &sc, const Frame &fr, const Levels &lv, const uint32_t i, Ray &ray, uint32_t &) const {
-    if (!PRIMARY) {
-      const float4 o = lv.ray_o[node_base - lv.offset[1] + i];
-      const float4 d = lv.ray_d[node_base - lv.offset[1] + i];
-      ray.o = mk(o.x, o.y, o.z);
-      ray.d = mk(d.x, d.y, d.z);
-      return true;
-    }
+  CRT_DI void ray(const DScene &, const Frame &, const Levels &lv, const uint32_t id, Ray &ray, float &) const {
+    const float4 o = lv.ray_o[id - lv.offset[1]], d = lv.ray_d[id - lv.offset[1]];
+    ray.o = mk(o.x, o.y, o.z);
+    ray.d = mk(d.x, d.y, d.z);
+  }
+  CRT_DI void answer(const DScene &, const Levels &lv, const uint32_t id, const Closest &cl) const {
+    lv.hit_tri[id] = cl.best_tri;
+    lv.hit_t[id] = cl.best_t;
+  }
+};
+
+// Level 0 of a frame: the pixel of the tile mapping and its camera ray, jittered in GI frames; answered into the frame's
+// hit records like the queue's rays.  The walk's JITTER is a template flag, so that the unsampled primary kernels keep
+// their register allocation; k_coop tests fr.gi at run time, so one k_coop serves both.  The level stays a kernel
+// parameter: k_shade / k_resolve over camera rays run every level of a frame (levels > 0 read the queue, not the source).
+struct CameraRays : QueueRays {
+  template <bool JITTER>
+  CRT_DI uint32_t items(const Frame &fr, const Levels &, const uint32_t) const { return level0_items<JITTER>(fr); }
+  template <bool JITTER>
+  CRT_DI bool take(const DScene &sc, const Frame &fr, const Levels &, const uint32_t, const uint32_t i, Ray &ray) const {
     uint32_t row, col;
     if (!item_pixel<JITTER>(fr, sc, fr.item_begin + i, row, col)) return false;
     if (JITTER)
@@ -567,37 +603,84 @@ struct ClosestWalk {
       primary_ray(fr.cam, sc.width, sc.height, row, col, ray.o, ray.d);
     return true;
   }
-  CRT_DI void begin(const Ray &, const uint32_t i, uint32_t &node) {
+  CRT_DI void ray(const DScene &sc, const Frame &fr, const Levels &lv, const uint32_t id, Ray &ray, float &) const {
+    uint32_t row, col;
+    item_pixel<true>(fr, sc, fr.item_begin + (id - lv.offset[0]), row, col);  // valid: the main kernel started this ray
+    if (fr.gi)
+      jittered_primary_ray(fr, sc.width, sc.height, row, col, ray.o, ray.d);
+    else
+      primary_ray(fr.cam, sc.width, sc.height, row, col, ray.o, ray.d);
+  }
+  template <bool GI>
+  CRT_DI bool valid(const DScene &sc, const Frame &fr, const uint32_t i) const {
+    uint32_t row, col;
+    return item_pixel<GI>(fr, sc, fr.item_begin + i, row, col);
+  }
+  // (keeps the statement structure k_shade had before the sources existed: the register allocation of k_shade<false>
+  // depends on it)
+  template <bool GI>
+  CRT_DI void level0(const DScene &sc, const Frame &fr, const uint32_t i, bool &valid, V3 &o, V3 &d, uint32_t &key,
+                     uint32_t &pix, uint32_t &n) const {
+    uint32_t row, col;
+    valid = item_pixel<GI>(fr, sc, fr.item_begin + i, row, col);
+    if (valid) {
+      if (GI) {
+        key = jittered_primary_ray(fr, sc.width, sc.height, row, col, o, d);
+        pix = row * sc.width + col;
+      } else {
+        primary_ray(fr.cam, sc.width, sc.height, row, col, o, d);
+      }
+      n++;
+    }
+  }
+  CRT_DI uint32_t ray_stat() const { return CRT_STAT_RAYS_PRIMARY; }
+};
+
+// A closest-hit walk over the rays of source Src; the answer is the closest hit of the ray.
+template <bool P, bool JITTER, class Src>
+struct ClosestWalk {
+  static constexpr bool PRIMARY = P, SHADOW = false;
+  static constexpr uint32_t STAT_NODES = CRT_STAT_NODES_CLOSEST, STAT_TRIS = CRT_STAT_TRIS_CLOSEST;
+  const uint32_t level, total, base;
+  Closest cl;
+  const DScene &sc;
+  const Src &src;
+  CRT_DI ClosestWalk(const DScene &s, const Frame &fr, const Levels &lv, const uint32_t lvl, const Src &r)
+      : level(r.level(lvl)), total(r.template items<JITTER>(fr, lv, level)), base(r.base(lv, level)), sc(s), src(r) {
     closest_begin(cl);
-    node = node_base + i;
+  }
+  CRT_DI bool take(const DScene &s, const Frame &fr, const Levels &lv, const uint32_t i, Ray &ray, uint32_t &) const {
+    return src.template take<JITTER>(s, fr, lv, base, i, ray);
+  }
+  CRT_DI void begin(const Ray &, const uint32_t i, uint32_t &id) {
+    closest_begin(cl);
+    id = base + i;
   }
   CRT_DI float tri_dist() const { return 0.f; }
   // conservative culling: beyond the best finite hit; behind the origin once a finite hit exists (crt_device.cuh)
   CRT_DI float limit() const { return cl.min_t; }
   CRT_DI bool allow_behind() const { return cl.min_t < CRT_INF; }
   template <bool COUNT>
-  CRT_DI bool tri(const DScene &sc, WarpShare &ws, const bool parked, const bool flush, Trav &tv, uint32_t &n_tris) {
+  CRT_DI bool tri(const DScene &s, WarpShare &ws, const bool parked, const bool flush, Trav &tv, uint32_t &n_tris) {
     bool dummy = false;
-    tri_phase<false, PRIMARY, COUNT>(sc, ws, parked, flush, tv.tref, tv.tend, cl, dummy, n_tris);
+    tri_phase<false, PRIMARY, COUNT>(s, ws, parked, flush, tv.tref, tv.tend, cl, dummy, n_tris);
     return false;
   }
-  CRT_DI void answer(const Levels &lv, const uint32_t node) const {
-    lv.hit_tri[node] = cl.best_tri;
-    lv.hit_t[node] = cl.best_t;
-  }
-  CRT_DI bool handoff(const Levels &lv, const bool want, const uint32_t node, const Trav &tv, bool &closed) const {
-    return tail_handoff(lv, level, want, node, tv, cl.best_t, cl.best_tri, closed);
+  CRT_DI void answer(const Levels &lv, const uint32_t id) const { src.answer(sc, lv, id, cl); }
+  CRT_DI bool handoff(const Levels &lv, const bool want, const uint32_t id, const Trav &tv, bool &closed) const {
+    return tail_handoff(lv, level, want, id, tv, cl.best_t, cl.best_tri, closed);
   }
   CRT_DI void finish(const Levels &) const {}
 };
 
-template <bool PRIMARY, bool COUNT, int REFILL, int MODE, bool CULL, bool WIDE, bool JITTER = false>
-__global__ void __launch_bounds__(CRT_TRAV_BLOCK, PRIMARY ? CRT_TRAV_MIN_BLOCKS : CRT_TRAV_MIN_BLOCKS_SEC) k_closest(const DScene sc, const Frame fr, const Levels lv, const uint32_t level,
-                                                uint32_t *__restrict__ work_counter) {
+// Work item = one ray of src at `level`; PRIMARY: the primary ray's back-face rule (Ray.cpp:13).
+template <class Src, bool PRIMARY, bool COUNT, int REFILL, int MODE, bool CULL, bool WIDE, bool JITTER = false>
+__global__ void __launch_bounds__(CRT_TRAV_BLOCK, std::is_same<Src, QueueRays>::value ? CRT_TRAV_MIN_BLOCKS_SEC : CRT_TRAV_MIN_BLOCKS)
+    k_closest(const DScene sc, const Frame fr, const Levels lv, const uint32_t level, uint32_t *__restrict__ work_counter, const Src src) {
   static_assert(MODE == 2, "only loop mode 2 is implemented");
   __shared__ WarpShare s_ws[CRT_TRAV_BLOCK / 32];
   WarpShare &ws = s_ws[threadIdx.x >> 5];
-  ClosestWalk<PRIMARY, JITTER> w(fr, lv, level);
+  ClosestWalk<PRIMARY, JITTER, Src> w(sc, fr, lv, level, src);
   walk_loop<REFILL, CULL, WIDE, false, (COUNT ? 0 : (WIDE ? 2 : 1)), COUNT, !COUNT, false>(sc, fr, lv, work_counter, ws, w);
 }
 
@@ -657,37 +740,6 @@ static __device__ __noinline__ void spawn_diffuse(const Frame &fr, const Levels 
   }
 }
 
-// Where level 0 of k_shade / k_resolve comes from (the caller's rays: RaysLevel0, with the shade kernels at the end):
-//   valid(sc, fr, i)                    level-0 slot i holds a ray
-//   ray<GI>(sc, fr, i, valid, o, d, key, pix, n)  valid: slot i holds a ray; then its ray, GI: its root path key and
-//                                                 pixel index, and n += 1
-//   stat()                              the CRT_STAT_RAYS_* slot its rays count in
-// CameraLevel0: the pixel of the tile mapping and its (jittered) camera ray.  (ray() keeps the statement structure
-// k_shade had before the sources existed: the register allocation of k_shade<false> depends on it.)
-struct CameraLevel0 {
-  template <bool GI>
-  CRT_DI bool valid(const DScene &sc, const Frame &fr, const uint32_t i) const {
-    uint32_t row, col;
-    return item_pixel<GI>(fr, sc, fr.item_begin + i, row, col);
-  }
-  template <bool GI>
-  CRT_DI void ray(const DScene &sc, const Frame &fr, const uint32_t i, bool &valid, V3 &o, V3 &d, uint32_t &key,
-                  uint32_t &pix, uint32_t &n) const {
-    uint32_t row, col;
-    valid = item_pixel<GI>(fr, sc, fr.item_begin + i, row, col);
-    if (valid) {
-      if (GI) {
-        key = jittered_primary_ray(fr, sc.width, sc.height, row, col, o, d);
-        pix = row * sc.width + col;
-      } else {
-        primary_ray(fr.cam, sc.width, sc.height, row, col, o, d);
-      }
-      n++;
-    }
-  }
-  CRT_DI uint32_t stat() const { return CRT_STAT_RAYS_PRIMARY; }
-};
-
 // GI: frames under the sampling contract (crt_sampling.h): jittered level 0, path keys carried in ray_o.w / pixel index in
 // ray_d.w, and every diffuse hit also spawns G diffuse children (COMB_GI).  GI = false is the unsampled kernel.
 template <bool GI, class L0>
@@ -703,7 +755,7 @@ CRT_DI void shade_level(const DScene &sc, const Frame &fr, const Levels &lv, con
     uint32_t key = 0, pix = 0;  // GI: path key of this ray, global pixel index
     if (valid) {
       if (level == 0) {
-        src.template ray<GI>(sc, fr, i, valid, o, d, key, pix, n_prim);
+        src.template level0<GI>(sc, fr, i, valid, o, d, key, pix, n_prim);
       } else {
         const float4 ro = lv.ray_o[node - lv.offset[1]];
         const float4 rd = lv.ray_d[node - lv.offset[1]];
@@ -847,15 +899,16 @@ CRT_DI void shade_level(const DScene &sc, const Frame &fr, const Levels &lv, con
     }
   }
   // ray statistics (traced rays only, SURVEY 8(d)); n_prim: level-0 rays, counted under the source's type
-  warp_stat_add(lv, src.stat(), (unsigned long long)n_prim);
+  warp_stat_add(lv, src.ray_stat(), (unsigned long long)n_prim);
   warp_stat_add(lv, CRT_STAT_RAYS_REFLECTION, (unsigned long long)n_refl);
   warp_stat_add(lv, CRT_STAT_RAYS_REFRACTION, (unsigned long long)n_refr);
   if (GI) warp_stat_add(lv, CRT_STAT_DIFFUSE, (unsigned long long)n_diff);
 }
 
-template <bool GI>
-__global__ void __launch_bounds__(256) k_shade(const DScene sc, const Frame fr, const Levels lv, const uint32_t level) {
-  shade_level<GI>(sc, fr, lv, level, CameraLevel0{});
+// Level 0 reads src (CameraRays, ShadeRays), every other level the queue.
+template <bool GI, class Src>
+__global__ void __launch_bounds__(256) k_shade(const DScene sc, const Frame fr, const Levels lv, const uint32_t level, const Src src) {
+  shade_level<GI>(sc, fr, lv, src.level(level), src);
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -889,17 +942,17 @@ CRT_DI float shadow_limit(const Ray &ray, const float dist) {
   return dist * 1.0001f + 1e-4f + 1e-6f * (fabsf(ray.o.x) + fabsf(ray.o.y) + fabsf(ray.o.z));
 }
 
-// ZERO_TERMS: a pair whose light term is exactly zero may be answered without a walk (not in the visit-all counting mode)
-template <bool ZERO_TERMS>
-struct ShadowWalk {
-  static constexpr bool PRIMARY = false, SHADOW = true;
-  static constexpr uint32_t STAT_NODES = CRT_STAT_NODES_SHADOW, STAT_TRIS = CRT_STAT_TRIS_SHADOW;
-  const uint32_t n_hits, total;
-  uint32_t n_moot = 0;
-  float dist = 0.0f, t_limit = 0.0f;
-  bool occluded = false;
-  CRT_DI ShadowWalk(const DScene &sc, const Levels &lv) : n_hits(lv.counts[CRT_MAX_LEVELS]), total(n_hits * sc.n_lights) {}
-  CRT_DI bool take(const DScene &sc, const Frame &fr, const Levels &lv, const uint32_t i, Ray &ray, uint32_t &slot) {
+// The diffuse hits of a frame towards each light: item i = pair (hit i % n_hits, light i / n_hits), record id = its
+// visibility slot hit * n_lights + light.  ZERO_TERMS: a pair whose light term is exactly zero may be answered without
+// a walk (not in the visit-all counting mode).
+struct ShadowPairs {
+  static constexpr bool SHADOW = true;
+  CRT_DI uint32_t level(const uint32_t l) const { return l; }
+  CRT_DI uint32_t base(const Levels &lv) const { return lv.counts[CRT_MAX_LEVELS]; }  // n_hits
+  CRT_DI uint32_t items(const DScene &sc, const uint32_t n_hits) const { return n_hits * sc.n_lights; }
+  template <bool ZERO_TERMS>
+  CRT_DI bool take(const DScene &sc, const Frame &fr, const Levels &lv, const uint32_t n_hits, const uint32_t i, Ray &ray,
+                   float &dist, uint32_t &slot, uint32_t &n_moot) const {
     const uint32_t light = i / n_hits, hit = i - light * n_hits;
     const float4 q0 = lv.dq[3 * (size_t)hit], q1 = lv.dq[3 * (size_t)hit + 1];
     float contrib;
@@ -922,8 +975,33 @@ struct ShadowWalk {
     }
     return !moot;
   }
+  CRT_DI void ray(const DScene &sc, const Frame &fr, const Levels &lv, const uint32_t id, Ray &ray, float &dist) const {
+    const uint32_t hit = id / sc.n_lights, light = id - hit * sc.n_lights;
+    const float4 q0 = lv.dq[3 * (size_t)hit], q1 = lv.dq[3 * (size_t)hit + 1];
+    float contrib;
+    shadow_ray_setup(sc, fr, mk(q0.x, q0.y, q0.z), mk(q1.x, q1.y, q1.z), light, ray, dist, contrib);
+  }
+  CRT_DI float limit(const Ray &ray, const float dist) const { return shadow_limit(ray, dist); }
+  CRT_DI void answer(const Levels &lv, const uint32_t id, const bool occluded) const { lv.vis[id] = occluded ? 0 : 1; }
+  CRT_DI void declined(const Levels &lv, const uint32_t n) const { warp_stat_add(lv, CRT_STAT_ZERO_TERM, n); }
+};
+
+// A shadow walk over the rays of source Src; the answer is whether a candidate lies within the ray's distance bound.
+template <bool ZERO_TERMS, class Src>
+struct ShadowWalk {
+  static constexpr bool PRIMARY = false, SHADOW = true;
+  static constexpr uint32_t STAT_NODES = CRT_STAT_NODES_SHADOW, STAT_TRIS = CRT_STAT_TRIS_SHADOW;
+  const uint32_t base, total;
+  uint32_t n_declined = 0;
+  float dist = 0.0f, t_limit = 0.0f;
+  bool occluded = false;
+  const Src &src;
+  CRT_DI ShadowWalk(const DScene &sc, const Levels &lv, const Src &r) : base(r.base(lv)), total(r.items(sc, base)), src(r) {}
+  CRT_DI bool take(const DScene &sc, const Frame &fr, const Levels &lv, const uint32_t i, Ray &ray, uint32_t &id) {
+    return src.template take<ZERO_TERMS>(sc, fr, lv, base, i, ray, dist, id, n_declined);
+  }
   CRT_DI void begin(const Ray &ray, const uint32_t, uint32_t &) {
-    t_limit = shadow_limit(ray, dist);
+    t_limit = src.limit(ray, dist);
     occluded = false;
   }
   CRT_DI float tri_dist() const { return dist; }
@@ -935,22 +1013,22 @@ struct ShadowWalk {
     tri_phase<true, false, COUNT>(sc, ws, parked, flush, tv.tref, tv.tend, unused, occluded, n_tris);
     return occluded;
   }
-  CRT_DI void answer(const Levels &lv, const uint32_t slot) const { lv.vis[slot] = occluded ? 0 : 1; }
-  CRT_DI bool handoff(const Levels &lv, const bool want, const uint32_t slot, const Trav &tv, bool &closed) const {
-    return tail_handoff(lv, CRT_MAX_LEVELS, want, slot, tv, 0.0f, CRT_INVALID, closed);
+  CRT_DI void answer(const Levels &lv, const uint32_t id) const { src.answer(lv, id, occluded); }
+  CRT_DI bool handoff(const Levels &lv, const bool want, const uint32_t id, const Trav &tv, bool &closed) const {
+    return tail_handoff(lv, CRT_MAX_LEVELS, want, id, tv, 0.0f, CRT_INVALID, closed);
   }
-  CRT_DI void finish(const Levels &lv) const { warp_stat_add(lv, CRT_STAT_ZERO_TERM, n_moot); }
+  CRT_DI void finish(const Levels &lv) const { src.declined(lv, n_declined); }
 };
 
 // SKIPR: shadow rays ignore refractive meshes, as the reference does only when !useGI (AccelerationStructure.cpp:67-71);
 // GI frames instantiate SKIPR = false.
-template <int COUNT, int REFILL, int MODE, bool CULL, bool WIDE, bool SKIPR = true>
+template <class Src, int COUNT, int REFILL, int MODE, bool CULL, bool WIDE, bool SKIPR = true>
 __global__ void __launch_bounds__(CRT_TRAV_BLOCK, CRT_TRAV_MIN_BLOCKS) k_shadow(const DScene sc, const Frame fr, const Levels lv,
-                                                                             uint32_t *__restrict__ work_counter) {
+                                                                             uint32_t *__restrict__ work_counter, const Src src) {
   static_assert(MODE == 2, "only loop mode 2 is implemented");
   __shared__ WarpShare s_ws[CRT_TRAV_BLOCK / 32];
   WarpShare &ws = s_ws[threadIdx.x >> 5];
-  ShadowWalk<COUNT != 1> w(sc, lv);
+  ShadowWalk<COUNT != 1, Src> w(sc, lv, src);
   walk_loop<REFILL, CULL, WIDE, SKIPR, (COUNT == 1 ? 0 : (WIDE ? 2 : 1)), (COUNT != 0), COUNT == 0, COUNT != 1>(
       sc, fr, lv, work_counter, ws, w);
 }
@@ -1062,45 +1140,12 @@ __global__ void k_mark(uint32_t *flag) {
   if (threadIdx.x == 0) *reinterpret_cast<volatile uint32_t *>(flag) = 1u;
 }
 
-// Where k_coop's walks come from and where their answers go (the ray source of coop_walks):
-//   ray<SHADOW, PRIMARY>(sc, lv, id, ray, dist)  the ray of record id (and, SHADOW, its distance bound)
-//   shadow_limit(ray, dist)                      the culling bound of a shadow walk (CULL)
-//   shadow_answer(lv, id, occluded)              closest_answer(sc, lv, id, cl)
-// CoopFrameSrc: the walks of a frame's traversal launches (queue nodes / visibility slots); CoopQuerySrc (below, with
-// the query kernels): a caller's ray batch.
-struct CoopFrameSrc {
-  const Frame &fr;
-  template <bool SHADOW, bool PRIMARY>
-  CRT_DI void ray(const DScene &sc, const Levels &lv, const uint32_t id, Ray &ray, float &dist) const {
-    if (SHADOW) {
-      const uint32_t hit = id / sc.n_lights, light = id - hit * sc.n_lights;
-      const float4 q0 = lv.dq[3 * (size_t)hit], q1 = lv.dq[3 * (size_t)hit + 1];
-      float contrib;
-      shadow_ray_setup(sc, fr, mk(q0.x, q0.y, q0.z), mk(q1.x, q1.y, q1.z), light, ray, dist, contrib);
-    } else if (PRIMARY) {
-      uint32_t row, col;
-      item_pixel<true>(fr, sc, fr.item_begin + (id - lv.offset[0]), row, col);  // valid: the main kernel started this ray
-      if (fr.gi)
-        jittered_primary_ray(fr, sc.width, sc.height, row, col, ray.o, ray.d);
-      else
-        primary_ray(fr.cam, sc.width, sc.height, row, col, ray.o, ray.d);
-    } else {
-      const float4 o = lv.ray_o[id - lv.offset[1]], d = lv.ray_d[id - lv.offset[1]];
-      ray.o = mk(o.x, o.y, o.z);
-      ray.d = mk(d.x, d.y, d.z);
-    }
-  }
-  CRT_DI float shadow_limit(const Ray &ray, const float dist) const { return crtd::shadow_limit(ray, dist); }
-  CRT_DI void shadow_answer(const Levels &lv, const uint32_t id, const bool occluded) const { lv.vis[id] = occluded ? 0 : 1; }
-  CRT_DI void closest_answer(const DScene &, const Levels &lv, const uint32_t id, const Closest &cl) const {
-    lv.hit_tri[id] = cl.best_tri;
-    lv.hit_t[id] = cl.best_t;
-  }
-};
-
-// The body of k_coop and k_coop_query.  SKIPR: shadow rays ignore refractive meshes (false in GI frames, see k_shadow)
+// The body of k_coop.  Its walks come from, and their answers go to, the ray source of the traversal kernel that handed
+// them off: src.ray rebuilds the ray of a record, src.limit bounds a shadow walk, src.answer writes the answer.
+// SKIPR: shadow rays ignore refractive meshes (false in GI frames, see k_shadow)
 template <bool SHADOW, bool PRIMARY, bool CULL, int GW, bool SKIPR, class Src>
-CRT_DI void coop_walks(const DScene &sc, const Levels &lv, const uint32_t level, const uint32_t early, WarpCoop &wc, const Src &src) {
+CRT_DI void coop_walks(const DScene &sc, const Frame &fr, const Levels &lv, const uint32_t level, const uint32_t early, WarpCoop &wc,
+                       const Src &src) {
   constexpr uint32_t NG = 32u / GW;            // walks per warp
   constexpr uint32_t CAP = CRT_COOP_CAP / NG;  // LIFO entries per walk
   static_assert(GW == 8 || GW == 16 || GW == 32, "group width");
@@ -1161,7 +1206,7 @@ CRT_DI void coop_walks(const DScene &sc, const Levels &lv, const uint32_t level,
       } else if (got != CRT_INVALID) {
         const uint4 r0 = __ldcg(&lv.ovf[3 * (size_t)r]), r1 = __ldcg(&lv.ovf[3 * (size_t)r + 1]), r2 = __ldcg(&lv.ovf[3 * (size_t)r + 2]);
         id = got;
-        src.template ray<SHADOW, PRIMARY>(sc, lv, id, ray, dist);
+        src.ray(sc, fr, lv, id, ray, dist);
         ray_prepare(ray, PRIMARY);
         // the walk's state where the main kernel left it
         cur = r0.y;
@@ -1175,7 +1220,10 @@ CRT_DI void coop_walks(const DScene &sc, const Levels &lv, const uint32_t level,
         cl.best_t = __uint_as_float(r2.z);
         cl.best_tri = r2.w;
         cl.min_t = (cl.best_tri != CRT_INVALID && cl.best_t < CRT_INF) ? cl.best_t : CRT_INF;
-        lim = SHADOW ? src.shadow_limit(ray, dist) : cl.min_t;
+        if constexpr (SHADOW)
+          lim = src.limit(ray, dist);
+        else
+          lim = cl.min_t;
         occluded = false;
         in_mesh = false;
         busy = true;
@@ -1244,10 +1292,10 @@ CRT_DI void coop_walks(const DScene &sc, const Levels &lv, const uint32_t level,
       } else {
         // itinerary complete
         if (gl == 0) {
-          if (SHADOW)
-            src.shadow_answer(lv, id, false);
+          if constexpr (SHADOW)
+            src.answer(lv, id, false);
           else
-            src.closest_answer(sc, lv, id, cl);
+            src.answer(sc, lv, id, cl);
         }
         busy = false;
       }
@@ -1359,7 +1407,9 @@ CRT_DI void coop_walks(const DScene &sc, const Levels &lv, const uint32_t level,
         }
       }
       if (SHADOW && occluded) {  // the first occluder ends the record (SURVEY App. A-11)
-        if (gl == 0) src.shadow_answer(lv, id, true);
+        if constexpr (SHADOW) {
+          if (gl == 0) src.answer(lv, id, true);
+        }
         busy = false;
         in_mesh = false;
         __syncwarp(gm);
@@ -1379,10 +1429,12 @@ CRT_DI void coop_walks(const DScene &sc, const Levels &lv, const uint32_t level,
 #endif
 }
 
-template <bool SHADOW, bool PRIMARY, bool CULL, int GW, bool SKIPR = true>
-__global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_coop(const DScene sc, const Frame fr, const Levels lv, const uint32_t level, const uint32_t early) {
+// k_coop over the walks k_closest / k_shadow handed off from the rays of src at `level`
+template <class Src, bool PRIMARY, bool CULL, int GW, bool SKIPR = true>
+__global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_coop(const DScene sc, const Frame fr, const Levels lv, const uint32_t level,
+                                                                                 const uint32_t early, const Src src) {
   __shared__ WarpCoop s_wc[CRT_COOP_WARPS];
-  coop_walks<SHADOW, PRIMARY, CULL, GW, SKIPR>(sc, lv, level, early, s_wc[threadIdx.x >> 5], CoopFrameSrc{fr});
+  coop_walks<Src::SHADOW, PRIMARY, CULL, GW, SKIPR>(sc, fr, lv, src.level(level), early, s_wc[threadIdx.x >> 5], src);
 }
 
 // K3c: the light loop of RayTracer::calculateDiffusion (RayTracer.cpp:308-330): per diffuse hit, walk the lights IN
@@ -1449,9 +1501,9 @@ CRT_DI void resolve_level(const DScene &sc, const Frame &fr, const Levels &lv, c
   }
 }
 
-template <bool GI>
-__global__ void __launch_bounds__(256) k_resolve(const DScene sc, const Frame fr, const Levels lv, const uint32_t level) {
-  resolve_level<GI>(sc, fr, lv, level, CameraLevel0{});
+template <bool GI, class Src>
+__global__ void __launch_bounds__(256) k_resolve(const DScene sc, const Frame fr, const Levels lv, const uint32_t level, const Src src) {
+  resolve_level<GI>(sc, fr, lv, src.level(level), src);
 }
 
 // Sample pass fr.sample of a GI frame: acc = acc + c_s in sample order (acc starts at (0,0,0)); the last pass leaves
@@ -1875,8 +1927,8 @@ __global__ void __launch_bounds__(256) k_generate_rays(const DScene sc, const DC
 // ------------------------------------------------------------------------------------------------------------
 // Caller-supplied ray batches (crtb200_trace_rays_device, DESIGN.md 3.12): RayTracer::trace (RayTracer.cpp:453-458) and
 // the non-GI RayTracer::hasIntersection (RayTracer.cpp:507-518) for rays the caller holds in device memory, walked by
-// the same persistent loop as K2 / K3 (walk kinds QueryClosestWalk / QueryShadowWalk) and handed off to the same k_coop
-// body (ray source CoopQuerySrc).  Work item i = ray i of the batch; its answer goes straight to the caller's arrays.
+// k_closest / k_shadow and handed off to k_coop with the sources QueryClosest / QueryShadow.  Work item i = ray i of the
+// batch = record id i; its answer goes straight to the caller's arrays.
 // ------------------------------------------------------------------------------------------------------------
 struct QueryBatch {
   const float *rays;          // n x 6: origin xyz, direction xyz
@@ -1914,220 +1966,106 @@ CRT_DI void query_store_hit(const DScene &sc, HitRec *hits, const uint32_t i, co
   hits[i] = h;
 }
 
-// Closest hit of ray i; PRIMARY (CRTB200_RAY_PRIMARY): the primary ray's back-face rule (Ray.cpp:13).  Limits as
-// ClosestWalk's: culling in parameter space holds for any direction length (DESIGN.md 3.12).
-template <bool P>
-struct QueryClosestWalk {
-  static constexpr bool PRIMARY = P, SHADOW = false;
-  static constexpr uint32_t STAT_NODES = CRT_STAT_NODES_CLOSEST, STAT_TRIS = CRT_STAT_TRIS_CLOSEST;
-  const DScene &sc;
-  const QueryBatch &qb;
-  const uint32_t total;
-  Closest cl;
-  CRT_DI QueryClosestWalk(const DScene &s, const QueryBatch &b) : sc(s), qb(b), total(b.n) { closest_begin(cl); }
-  CRT_DI bool take(const DScene &, const Frame &, const Levels &, const uint32_t i, Ray &ray, uint32_t &) const {
-    query_ray(qb.rays, i, ray);
+// Closest hit of ray i (the walk's PRIMARY: CRTB200_RAY_PRIMARY batches).  Limits as the frame's: culling in parameter
+// space holds for any direction length (DESIGN.md 3.12).
+struct QueryClosest : QueryBatch {
+  static constexpr bool SHADOW = false;
+  CRT_DI uint32_t level(const uint32_t) const { return 0u; }
+  template <bool>
+  CRT_DI uint32_t items(const Frame &, const Levels &, const uint32_t) const { return n; }
+  CRT_DI uint32_t base(const Levels &, const uint32_t) const { return 0u; }
+  template <bool>
+  CRT_DI bool take(const DScene &, const Frame &, const Levels &, const uint32_t, const uint32_t i, Ray &ray) const {
+    query_ray(rays, i, ray);
     return true;
   }
-  CRT_DI void begin(const Ray &, const uint32_t i, uint32_t &id) {
-    closest_begin(cl);
-    id = i;
+  CRT_DI void ray(const DScene &, const Frame &, const Levels &, const uint32_t id, Ray &ray, float &) const { query_ray(rays, id, ray); }
+  CRT_DI void answer(const DScene &sc, const Levels &, const uint32_t id, const Closest &cl) const {
+    query_store_hit(sc, hits, id, cl.best_tri, cl.best_t);
   }
-  CRT_DI float tri_dist() const { return 0.f; }
-  CRT_DI float limit() const { return cl.min_t; }
-  CRT_DI bool allow_behind() const { return cl.min_t < CRT_INF; }
-  template <bool COUNT>
-  CRT_DI bool tri(const DScene &s, WarpShare &ws, const bool parked, const bool flush, Trav &tv, uint32_t &n_tris) {
-    bool dummy = false;
-    tri_phase<false, PRIMARY, COUNT>(s, ws, parked, flush, tv.tref, tv.tend, cl, dummy, n_tris);
-    return false;
-  }
-  CRT_DI void answer(const Levels &, const uint32_t i) const { query_store_hit(sc, qb.hits, i, cl.best_tri, cl.best_t); }
-  CRT_DI bool handoff(const Levels &lv, const bool want, const uint32_t i, const Trav &tv, bool &closed) const {
-    return tail_handoff(lv, 0u, want, i, tv, cl.best_t, cl.best_tri, closed);
-  }
-  CRT_DI void finish(const Levels &) const {}
 };
 
 // Any hit of ray i within max_distance[i]: occluded iff some candidate has |P - o| <= max_distance (refractive meshes
 // skipped, AccelerationStructure.cpp:67-74).  A query has no light term, so no walk is skipped for a zero term.
-struct QueryShadowWalk {
-  static constexpr bool PRIMARY = false, SHADOW = true;
-  static constexpr uint32_t STAT_NODES = CRT_STAT_NODES_SHADOW, STAT_TRIS = CRT_STAT_TRIS_SHADOW;
-  const QueryBatch &qb;
-  const uint32_t total;
-  float dist = 0.0f, t_limit = 0.0f;
-  bool occluded = false;
-  CRT_DI explicit QueryShadowWalk(const QueryBatch &b) : qb(b), total(b.n) {}
-  CRT_DI bool take(const DScene &, const Frame &, const Levels &, const uint32_t i, Ray &ray, uint32_t &) {
-    query_ray(qb.rays, i, ray);
-    dist = qb.max_distance[i];
+struct QueryShadow : QueryBatch {
+  static constexpr bool SHADOW = true;
+  CRT_DI uint32_t level(const uint32_t) const { return 0u; }
+  CRT_DI uint32_t base(const Levels &) const { return 0u; }
+  CRT_DI uint32_t items(const DScene &, const uint32_t) const { return n; }
+  template <bool>
+  CRT_DI bool take(const DScene &, const Frame &, const Levels &, const uint32_t, const uint32_t i, Ray &ray, float &dist,
+                   uint32_t &id, uint32_t &) const {
+    query_ray(rays, i, ray);
+    dist = max_distance[i];
+    id = i;
     return true;
   }
-  CRT_DI void begin(const Ray &ray, const uint32_t i, uint32_t &id) {
-    t_limit = query_shadow_limit(ray, dist);
-    occluded = false;
-    id = i;
+  CRT_DI void ray(const DScene &, const Frame &, const Levels &, const uint32_t id, Ray &ray, float &dist) const {
+    query_ray(rays, id, ray);
+    dist = max_distance[id];
   }
-  CRT_DI float tri_dist() const { return dist; }
-  CRT_DI float limit() const { return t_limit; }
-  CRT_DI bool allow_behind() const { return true; }
-  template <bool COUNT>
-  CRT_DI bool tri(const DScene &sc, WarpShare &ws, const bool parked, const bool flush, Trav &tv, uint32_t &n_tris) {
-    Closest unused;
-    tri_phase<true, false, COUNT>(sc, ws, parked, flush, tv.tref, tv.tend, unused, occluded, n_tris);
-    return occluded;
-  }
-  CRT_DI void answer(const Levels &, const uint32_t i) const { qb.occluded[i] = occluded ? 1 : 0; }
-  CRT_DI bool handoff(const Levels &lv, const bool want, const uint32_t i, const Trav &tv, bool &closed) const {
-    return tail_handoff(lv, CRT_MAX_LEVELS, want, i, tv, 0.0f, CRT_INVALID, closed);
-  }
-  CRT_DI void finish(const Levels &) const {}
+  CRT_DI float limit(const Ray &ray, const float dist) const { return query_shadow_limit(ray, dist); }
+  CRT_DI void answer(const Levels &, const uint32_t id, const bool occ) const { occluded[id] = occ ? 1 : 0; }
+  CRT_DI void declined(const Levels &, const uint32_t) const {}
 };
-
-// lv: the query's own Levels (stats, hand-off records and counters; no ray queues).  Flags as k_closest / k_shadow's.
-template <bool PRIMARY, bool COUNT, int REFILL, bool CULL, bool WIDE>
-__global__ void __launch_bounds__(CRT_TRAV_BLOCK, CRT_TRAV_MIN_BLOCKS) k_query_closest(const DScene sc, const Levels lv, const QueryBatch qb,
-                                                                                    uint32_t *__restrict__ work_counter) {
-  __shared__ WarpShare s_ws[CRT_TRAV_BLOCK / 32];
-  WarpShare &ws = s_ws[threadIdx.x >> 5];
-  const Frame fr{};
-  QueryClosestWalk<PRIMARY> w(sc, qb);
-  walk_loop<REFILL, CULL, WIDE, false, (COUNT ? 0 : (WIDE ? 2 : 1)), COUNT, !COUNT, false>(sc, fr, lv, work_counter, ws, w);
-}
-
-template <int COUNT, int REFILL, bool CULL, bool WIDE>
-__global__ void __launch_bounds__(CRT_TRAV_BLOCK, CRT_TRAV_MIN_BLOCKS) k_query_shadow(const DScene sc, const Levels lv, const QueryBatch qb,
-                                                                                   uint32_t *__restrict__ work_counter) {
-  __shared__ WarpShare s_ws[CRT_TRAV_BLOCK / 32];
-  WarpShare &ws = s_ws[threadIdx.x >> 5];
-  const Frame fr{};
-  QueryShadowWalk w(qb);
-  walk_loop<REFILL, CULL, WIDE, true, (COUNT == 1 ? 0 : (WIDE ? 2 : 1)), (COUNT != 0), COUNT == 0, COUNT != 1>(
-      sc, fr, lv, work_counter, ws, w);
-}
-
-// The ray source of k_coop_query: record id = ray id of the batch
-struct CoopQuerySrc {
-  const QueryBatch &qb;
-  template <bool SHADOW, bool PRIMARY>
-  CRT_DI void ray(const DScene &, const Levels &, const uint32_t id, Ray &ray, float &dist) const {
-    query_ray(qb.rays, id, ray);
-    if (SHADOW) dist = qb.max_distance[id];
-  }
-  CRT_DI float shadow_limit(const Ray &ray, const float dist) const { return query_shadow_limit(ray, dist); }
-  CRT_DI void shadow_answer(const Levels &, const uint32_t id, const bool occluded) const { qb.occluded[id] = occluded ? 1 : 0; }
-  CRT_DI void closest_answer(const DScene &sc, const Levels &, const uint32_t id, const Closest &cl) const {
-    query_store_hit(sc, qb.hits, id, cl.best_tri, cl.best_t);
-  }
-};
-
-// k_coop over the walks a query kernel handed off.  Hand-off implies culling (crtb200_trace_rays_device), so CULL = true.
-template <bool SHADOW, bool PRIMARY>
-__global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_coop_query(const DScene sc, const Levels lv, const QueryBatch qb,
-                                                                                       const uint32_t early) {
-  __shared__ WarpCoop s_wc[CRT_COOP_WARPS];
-  coop_walks<SHADOW, PRIMARY, true, CRT_COOP_GROUP, true>(sc, lv, 0u, early, s_wc[threadIdx.x >> 5], CoopQuerySrc{qb});
-}
 
 // ------------------------------------------------------------------------------------------------------------
 // Caller-supplied rays shaded through the frame pipeline (crtb200_shade_rays_device, DESIGN.md 3.13): RayTracer::shootRay
 // (RayTracer.cpp:419-451) for a batch of rays.  Level 0 of a chunk is ray item_begin + i of the batch instead of a
-// pixel; every later level, the shadow pass, k_accumulate and the resolve of levels > 0 are the frame's kernels.  Four
-// places derive a level-0 ray, each has a kernel of its own here: the closest-hit walk (k_closest_rays), its hand-off
-// (k_coop_rays), k_shade_rays and k_resolve_rays; k_store_rays writes colour i and hit i.
+// pixel: k_closest, k_coop, k_shade and k_resolve read it through the source ShadeRays; every later level, the shadow
+// pass and k_accumulate are the frame's.  k_store_rays writes colour i and hit i.
 // ------------------------------------------------------------------------------------------------------------
-struct ShadeRays {
-  const float *rays;     // this GPU's range of the batch: n x 6 (origin xyz, direction xyz)
-  float *rgb;            // n x 3
-  HitRec *hits;          // n, or null
-  uint32_t first_index;  // GI: pixel index p of ray 0 of the range
-  uint32_t stat;         // CRT_STAT_RAYS_* slot of the batch's ray type
-};
-
 // Ray `item` of the range with shootRay's normalisation of the direction (RayTracer.cpp:420), applied once: the walk,
 // its hand-off and k_shade read the same bits
-CRT_DI void shade_ray(const ShadeRays &sr, const uint32_t item, V3 &o, V3 &d) {
+CRT_DI void shade_ray(const float *rays, const uint32_t item, V3 &o, V3 &d) {
   Ray r;
-  query_ray(sr.rays, item, r);
+  query_ray(rays, item, r);
   o = r.o;
   d = vnorm(r.d);
 }
 
-struct RaysLevel0 {
-  const ShadeRays &sr;
+// This GPU's range of the batch; record id = level-0 queue node, answered into the frame's hit records.  Its
+// launches are level 0 only.
+struct ShadeRays {
+  const float *rays;     // n x 6 (origin xyz, direction xyz)
+  float *rgb;            // n x 3
+  HitRec *hits;          // n, or null
+  uint32_t first_index;  // GI: pixel index p of ray 0 of the range
+  uint32_t stat;         // CRT_STAT_RAYS_* slot of the batch's ray type
+
+  static constexpr bool SHADOW = false;
+  CRT_DI uint32_t level(const uint32_t) const { return 0u; }
+  template <bool>
+  CRT_DI uint32_t items(const Frame &fr, const Levels &, const uint32_t) const { return fr.n_items0; }
+  CRT_DI uint32_t base(const Levels &lv, const uint32_t level) const { return lv.offset[level]; }
+  template <bool>
+  CRT_DI bool take(const DScene &, const Frame &fr, const Levels &, const uint32_t, const uint32_t i, Ray &ray) const {
+    shade_ray(rays, fr.item_begin + i, ray.o, ray.d);
+    return true;
+  }
+  CRT_DI void ray(const DScene &, const Frame &fr, const Levels &lv, const uint32_t id, Ray &ray, float &) const {
+    shade_ray(rays, fr.item_begin + (id - lv.offset[0]), ray.o, ray.d);
+  }
+  CRT_DI void answer(const DScene &, const Levels &lv, const uint32_t id, const Closest &cl) const {
+    lv.hit_tri[id] = cl.best_tri;
+    lv.hit_t[id] = cl.best_t;
+  }
   template <bool GI>
   CRT_DI bool valid(const DScene &, const Frame &, const uint32_t) const { return true; }
   // GI: p = first_index + item, s = fr.sample, root path key = R(p, s, 0, 0).z (the word jittered_primary_ray returns)
   template <bool GI>
-  CRT_DI void ray(const DScene &, const Frame &fr, const uint32_t i, bool &valid, V3 &o, V3 &d, uint32_t &key,
-                  uint32_t &pix, uint32_t &n) const {
-    shade_ray(sr, fr.item_begin + i, o, d);
+  CRT_DI void level0(const DScene &, const Frame &fr, const uint32_t i, bool &valid, V3 &o, V3 &d, uint32_t &key,
+                     uint32_t &pix, uint32_t &n) const {
+    shade_ray(rays, fr.item_begin + i, o, d);
     if (GI) {
-      pix = sr.first_index + fr.item_begin + i;
+      pix = first_index + fr.item_begin + i;
       key = crt_s_philox(pix, fr.sample, 0u, 0u, fr.seed, fr.frame_index).z;
     }
     valid = true;
     n++;
   }
-  CRT_DI uint32_t stat() const { return sr.stat; }
+  CRT_DI uint32_t ray_stat() const { return stat; }
 };
-
-// Level 0's closest-hit walk: ClosestWalk over the chunk's n_items0 rays of the batch.  PRIMARY (CRTB200_RAY_PRIMARY
-// batches): the primary ray's back-face rule, independent of where the ray comes from.
-template <bool P>
-struct RaysClosestWalk : ClosestWalk<P, false> {
-  const uint32_t total;
-  const ShadeRays &sr;
-  CRT_DI RaysClosestWalk(const Frame &fr, const Levels &lv, const ShadeRays &s) : ClosestWalk<P, false>(fr, lv, 0u), total(fr.n_items0), sr(s) {}
-  CRT_DI bool take(const DScene &, const Frame &fr, const Levels &, const uint32_t i, Ray &ray, uint32_t &) const {
-    shade_ray(sr, fr.item_begin + i, ray.o, ray.d);
-    return true;
-  }
-};
-
-template <bool PRIMARY, bool COUNT, int REFILL, bool CULL, bool WIDE>
-__global__ void __launch_bounds__(CRT_TRAV_BLOCK, CRT_TRAV_MIN_BLOCKS) k_closest_rays(const DScene sc, const Frame fr, const Levels lv, const ShadeRays sr,
-                                                                                   uint32_t *__restrict__ work_counter) {
-  __shared__ WarpShare s_ws[CRT_TRAV_BLOCK / 32];
-  WarpShare &ws = s_ws[threadIdx.x >> 5];
-  RaysClosestWalk<PRIMARY> w(fr, lv, sr);
-  walk_loop<REFILL, CULL, WIDE, false, (COUNT ? 0 : (WIDE ? 2 : 1)), COUNT, !COUNT, false>(sc, fr, lv, work_counter, ws, w);
-}
-
-// The ray source of k_coop_rays: record id = level-0 queue node id
-struct CoopRaysSrc {
-  const Frame &fr;
-  const ShadeRays &sr;
-  template <bool SHADOW, bool PRIMARY>
-  CRT_DI void ray(const DScene &, const Levels &lv, const uint32_t id, Ray &ray, float &) const {
-    shade_ray(sr, fr.item_begin + (id - lv.offset[0]), ray.o, ray.d);
-  }
-  CRT_DI float shadow_limit(const Ray &ray, const float dist) const { return crtd::shadow_limit(ray, dist); }
-  CRT_DI void shadow_answer(const Levels &, const uint32_t, const bool) const {}
-  CRT_DI void closest_answer(const DScene &, const Levels &lv, const uint32_t id, const Closest &cl) const {
-    lv.hit_tri[id] = cl.best_tri;
-    lv.hit_t[id] = cl.best_t;
-  }
-};
-
-// k_coop over the level-0 walks k_closest_rays handed off
-template <bool PRIMARY, bool CULL>
-__global__ void __launch_bounds__(32 * CRT_COOP_WARPS, CRT_COOP_MIN_BLOCKS) k_coop_rays(const DScene sc, const Frame fr, const Levels lv, const ShadeRays sr,
-                                                                                      const uint32_t early) {
-  __shared__ WarpCoop s_wc[CRT_COOP_WARPS];
-  coop_walks<false, PRIMARY, CULL, CRT_COOP_GROUP, true>(sc, lv, 0u, early, s_wc[threadIdx.x >> 5], CoopRaysSrc{fr, sr});
-}
-
-template <bool GI>
-__global__ void __launch_bounds__(256) k_shade_rays(const DScene sc, const Frame fr, const Levels lv, const ShadeRays sr) {
-  shade_level<GI>(sc, fr, lv, 0u, RaysLevel0{sr});
-}
-
-template <bool GI>
-__global__ void __launch_bounds__(256) k_resolve_rays(const DScene sc, const Frame fr, const Levels lv, const ShadeRays sr) {
-  resolve_level<GI>(sc, fr, lv, 0u, RaysLevel0{sr});
-}
 
 // Colour i and hit i of the chunk's rays, in place of k_store: a warp's 32 colours leave as 24 16-byte stores when rgb is
 // 16-byte aligned (chunks start at multiples of 32 rays, so every full warp's 384 bytes are then aligned too).  Counts

@@ -404,13 +404,13 @@ static int add_gpu(crtb200_ctx *c, int device) {
   g.sm_count = prop.multiProcessorCount;
   if (g.stream.create(cudaStreamNonBlocking) != cudaSuccess) return fail(CRTB200_ERR_CUDA, "cudaStreamCreate / cudaEventCreate failed");
   int occ = 0;
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_closest<true, false, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, false, false>, CRT_TRAV_BLOCK, 0);
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_closest<CameraRays, true, false, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, false, false>, CRT_TRAV_BLOCK, 0);
   g.blocks_closest = std::max(1, occ) * g.sm_count;
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_closest<false, false, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, false, false>, CRT_TRAV_BLOCK, 0);
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_closest<QueueRays, false, false, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, false, false>, CRT_TRAV_BLOCK, 0);
   g.blocks_closest_sec = std::max(1, occ) * g.sm_count;
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_shadow<0, CRT_REFILL_SHADOW, CRT_LOOP_MODE, false, false>, CRT_TRAV_BLOCK, 0);
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_shadow<ShadowPairs, 0, CRT_REFILL_SHADOW, CRT_LOOP_MODE, false, false>, CRT_TRAV_BLOCK, 0);
   g.blocks_shadow = std::max(1, occ) * g.sm_count;
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_coop<true, false, true, CRT_COOP_GROUP>, 32 * CRT_COOP_WARPS, 0);
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_coop<ShadowPairs, false, true, CRT_COOP_GROUP>, 32 * CRT_COOP_WARPS, 0);
   g.blocks_coop = std::max(1, occ) * g.sm_count;
   if (const char *env = getenv("CRT_BLOCKS_PER_SM")) {  // tuning only (tools/): resident persistent CTAs per SM
     const int b = atoi(env);
@@ -1523,7 +1523,6 @@ static int check_device_ptr(const Gpu &g, const void *p, size_t align, const cha
 struct Flavour {
   uint32_t count_work;
   bool cull, handoff, gi, wide_closest, wide_shadow;
-  const ShadeRays *rays = nullptr;  // level 0 reads this range of a caller's rays (crtb200_shade_rays_device), not pixels
 };
 
 static Flavour frame_flavour(const Gpu &g, const crtb200_options *o, const crtb200_sampling &smp) {
@@ -1553,110 +1552,100 @@ static void as_const_count(uint32_t v, F &&f) {
   v == 1 ? f(std::integral_constant<int, 1>{}) : v == 2 ? f(std::integral_constant<int, 2>{}) : f(std::integral_constant<int, 0>{});
 }
 
-// k_closest of level `level`: PRIMARY at level 0, jittered in GI frames; level 0 of caller rays: k_closest_rays, PRIMARY
-// for primary batches
-static void launch_closest(const Gpu &g, const Flavour &fl, const Frame &fr, QueueSet &q, uint32_t level) {
-  const bool primary = level == 0;
-  if (fl.rays && primary) {
-    as_const(fl.count_work != 0, [&](auto count) { as_const(fl.cull, [&](auto cull) { as_const(fl.wide_closest, [&](auto wide) {
-      as_const(fl.rays->stat == CRT_STAT_RAYS_PRIMARY, [&](auto prim) {
-        if constexpr (!(count && wide))
-          k_closest_rays<prim, count, CRT_REFILL_CLOSEST, cull, wide>
-              <<<g.blocks_closest, CRT_TRAV_BLOCK, dyn_smem(g, CRT_TRAV_BLOCK), q.stream>>>(g.sc, fr, q.lv, *fl.rays, q.work);
-      }); }); }); });
-    return;
-  }
+// The launches of one traversal over the rays of `src` at `level` (k_closest or k_shadow, and k_coop) on st; primary:
+// the primary ray's back-face rule.  Sources run with the flags they can have: camera rays are primary and jittered in
+// GI frames, a frame's queue is neither, a caller's rays are never jittered; queries skip refractive meshes and hand off
+// only culled walks (hand-off implies culling).
+template <class Src>
+static void launch_closest(const Gpu &g, const Flavour &fl, const Frame &fr, QueueSet &q, uint32_t level, const Src &src,
+                           bool primary, int blocks, cudaStream_t st) {
+  constexpr bool camera = std::is_same<Src, CameraRays>::value, queue = std::is_same<Src, QueueRays>::value;
   as_const(fl.count_work != 0, [&](auto count) { as_const(fl.cull, [&](auto cull) { as_const(fl.wide_closest, [&](auto wide) {
-    as_const(primary, [&](auto prim) { as_const(primary && fl.gi, [&](auto jitter) {
-      if constexpr (!(count && wide) && (prim || !jitter))
-        k_closest<prim, count, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, cull, wide, jitter>
-            <<<primary ? g.blocks_closest : g.blocks_closest_sec, CRT_TRAV_BLOCK, dyn_smem(g, CRT_TRAV_BLOCK), q.stream>>>(
-                g.sc, fr, q.lv, level, q.work + CRT_CTL_STRIDE * level);
+    as_const(primary, [&](auto prim) { as_const(camera && fl.gi, [&](auto jitter) {
+      if constexpr (!(count && wide) && (camera ? prim : !jitter && !(queue && prim)))
+        k_closest<Src, prim, count, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, cull, wide, jitter>
+            <<<blocks, CRT_TRAV_BLOCK, dyn_smem(g, CRT_TRAV_BLOCK), st>>>(g.sc, fr, q.lv, level, q.work + CRT_CTL_STRIDE * level, src);
     }); }); }); }); });
 }
-// the shadow pass of one chunk; SKIPR = false in GI frames
-static void launch_shadow(const Gpu &g, const Flavour &fl, const Frame &fr, QueueSet &q) {
+// SKIPR = false in GI frames
+template <class Src>
+static void launch_shadow(const Gpu &g, const Flavour &fl, const Frame &fr, QueueSet &q, const Src &src, int blocks, cudaStream_t st) {
+  constexpr bool query = std::is_same<Src, QueryShadow>::value;
   as_const_count(fl.count_work, [&](auto count) { as_const(fl.cull, [&](auto cull) { as_const(fl.wide_shadow, [&](auto wide) {
     as_const(!fl.gi, [&](auto skipr) {
-      if constexpr (count != 1 || !(cull || wide))
-        k_shadow<count, CRT_REFILL_SHADOW, CRT_LOOP_MODE, cull, wide, skipr>
-            <<<g.blocks_shadow, CRT_TRAV_BLOCK, wide ? dyn_smem(g, CRT_TRAV_BLOCK) : 0, q.stream>>>(
-                g.sc, fr, q.lv, q.work + CRT_CTL_STRIDE * CRT_MAX_LEVELS);
+      if constexpr ((count != 1 || !(cull || wide)) && (skipr || !query))
+        k_shadow<Src, count, CRT_REFILL_SHADOW, CRT_LOOP_MODE, cull, wide, skipr>
+            <<<blocks, CRT_TRAV_BLOCK, wide ? dyn_smem(g, CRT_TRAV_BLOCK) : 0, st>>>(
+                g.sc, fr, q.lv, q.work + CRT_CTL_STRIDE * CRT_MAX_LEVELS, src);
     }); }); }); });
 }
-// k_coop over the walks the shadow pass or closest-hit level `level` handed off; SKIPR = false in GI shadow passes
-static void launch_coop(const Gpu &g, const Flavour &fl, const Frame &fr, QueueSet &q, bool shadow, uint32_t level,
-                        int blocks, cudaStream_t st, uint32_t early) {
-  if (fl.rays && !shadow && level == 0) {  // (k_coop's PRIMARY source would regenerate camera rays)
-    as_const(fl.rays->stat == CRT_STAT_RAYS_PRIMARY, [&](auto prim) { as_const(fl.cull, [&](auto cull) {
-      k_coop_rays<prim, cull><<<blocks, 32 * CRT_COOP_WARPS, 0, st>>>(g.sc, fr, q.lv, *fl.rays, early);
-    }); });
-    return;
-  }
-  as_const(shadow, [&](auto sh) { as_const(!shadow && level == 0, [&](auto prim) { as_const(fl.cull, [&](auto cull) {
-    as_const(!(shadow && fl.gi), [&](auto skipr) {
-      if constexpr (!(sh && prim) && (sh || skipr))
-        k_coop<sh, prim, cull, CRT_COOP_GROUP, skipr><<<blocks, 32 * CRT_COOP_WARPS, 0, st>>>(g.sc, fr, q.lv, level, early);
-    }); }); }); });
+template <class Src>
+static void launch_coop(const Gpu &g, const Flavour &fl, const Frame &fr, QueueSet &q, uint32_t level, const Src &src,
+                        bool primary, int blocks, cudaStream_t st, uint32_t early) {
+  constexpr bool shadow = Src::SHADOW, camera = std::is_same<Src, CameraRays>::value, queue = std::is_same<Src, QueueRays>::value;
+  constexpr bool query = std::is_same<Src, QueryClosest>::value || std::is_same<Src, QueryShadow>::value;
+  as_const(primary, [&](auto prim) { as_const(fl.cull, [&](auto cull) { as_const(!(shadow && fl.gi), [&](auto skipr) {
+    if constexpr (!(shadow && prim) && ((shadow && !query) || skipr) && (cull || !query) && (camera ? prim : !(queue && prim)))
+      k_coop<Src, prim, cull, CRT_COOP_GROUP, skipr><<<blocks, 32 * CRT_COOP_WARPS, 0, st>>>(g.sc, fr, q.lv, level, early, src);
+  }); }); });
 }
 
-// One traversal launch on st -- k_closest of level `level`, the shadow pass, or a query kernel -- and with hand-off
-// k_coop around it (DESIGN.md 3.8).  launch(stream, coop_blocks, early) enqueues the walk source's traversal kernel
-// (coop_blocks = 0) or its k_coop pass.  With an early pass (`early_ok`: one queue set, and not a secondary level of a
-// frame) the side stream is forked BEFORE the traversal kernel is launched; behind it k_mark marks the traversal kernel's
-// end, the early pass starts on the side stream (its blocks get SM resources as the traversal kernel's blocks exit)
-// and joins, and the final pass runs over what is left.
+// One traversal launch over the rays of `src` on st -- k_closest of level `level`, or k_shadow -- and with hand-off
+// k_coop around it (DESIGN.md 3.8).  blocks: the traversal kernel's grid.  With an early pass (`early_ok`: one queue
+// set, and not a secondary level of a frame) the side stream is forked BEFORE the traversal kernel is launched; behind
+// it k_mark marks the traversal kernel's end, the early pass starts on the side stream (its blocks get SM resources as
+// the traversal kernel's blocks exit) and joins, and the final pass runs over what is left.
 // timed: the context whose per-launch events time them (closest_ms, shadow_ms, coop_*_ms), null for none; a mark with a
 // kind (0 closest, 1 shadow, 2 / 3 their k_coop part) opens a span and the next mark closes it, collect_stats reads
 // them in pairs.
-template <typename Launch>
-static int traverse(Gpu &g, bool handoff, bool early_ok, QueueSet &q, cudaStream_t st, bool shadow, uint32_t level,
-                    crtb200_ctx *timed, uint32_t &launches, const Launch &launch) {
+template <class Src>
+static int traverse(Gpu &g, const Flavour &fl, bool early_ok, QueueSet &q, cudaStream_t st, const Frame &fr, uint32_t level,
+                    const Src &src, bool primary, int blocks, crtb200_ctx *timed, uint32_t &launches) {
+  constexpr bool shadow = Src::SHADOW;
   auto mark = [&](int kind) {
     if (timed && kind >= 0) timed->kev_kind.push_back(kind);
     return timed ? record_next_event(timed, st) : cudaSuccess;
   };
-  const bool early = handoff && g.coop_early > 0 && early_ok;
+  const bool early = fl.handoff && g.coop_early > 0 && early_ok;
   CUDA_TRY(mark(shadow ? 1 : 0));
   if (early) {
     CUDA_TRY(cudaEventRecord(q.coop_fork, st));
     CUDA_TRY(cudaStreamWaitEvent(q.coop_stream, q.coop_fork, 0));
   }
-  launch(st, 0, 0u);
-  if (handoff) {
+  if constexpr (shadow)
+    launch_shadow(g, fl, fr, q, src, blocks, st);
+  else
+    launch_closest(g, fl, fr, q, level, src, primary, blocks, st);
+  if (fl.handoff) {
     CUDA_TRY(mark(-1));
     CUDA_TRY(mark(shadow ? 3 : 2));
     if (early) {
       k_mark<<<1, 32, 0, st>>>(q.lv.ovf_ctl + CRT_CTL_STRIDE * (shadow ? (uint32_t)CRT_MAX_LEVELS : level) + 24u);
-      launch(q.coop_stream, g.sm_count * g.coop_early, 1u);
+      launch_coop(g, fl, fr, q, level, src, primary, g.sm_count * g.coop_early, q.coop_stream, 1u);
       CUDA_TRY(cudaEventRecord(q.coop_join, q.coop_stream));
       CUDA_TRY(cudaStreamWaitEvent(st, q.coop_join, 0));
       launches += 2;
     }
-    launch(st, g.blocks_coop, 0u);
+    launch_coop(g, fl, fr, q, level, src, primary, g.blocks_coop, st, 0u);
     launches++;
   }
   CUDA_TRY(mark(-1));
   return CRTB200_OK;
 }
 
-// traverse for k_closest of level `level` or the shadow pass of a frame's chunk
-static int traverse_frame(Gpu &g, const Flavour &fl, const Frame &fr, QueueSet &q, bool shadow, uint32_t level,
+// traverse for k_closest of level `level` (QueueRays, or the request's level-0 source) or the shadow pass (ShadowPairs)
+// of a frame's chunk
+template <class Src>
+static int traverse_frame(Gpu &g, const Flavour &fl, const Frame &fr, QueueSet &q, uint32_t level, const Src &src, bool primary,
                           crtb200_ctx *timed, uint32_t &launches) {
-  return traverse(g, fl.handoff, g.cap_sets == 1 && (shadow || level == 0), q, q.stream, shadow, level, timed, launches,
-                  [&](cudaStream_t st, int coop_blocks, uint32_t early) {
-                    if (coop_blocks)
-                      launch_coop(g, fl, fr, q, shadow, level, coop_blocks, st, early);
-                    else if (shadow)
-                      launch_shadow(g, fl, fr, q);
-                    else
-                      launch_closest(g, fl, fr, q, level);
-                  });
+  const int blocks = Src::SHADOW ? g.blocks_shadow : level == 0 ? g.blocks_closest : g.blocks_closest_sec;
+  return traverse(g, fl, g.cap_sets == 1 && (Src::SHADOW || level == 0), q, q.stream, fr, level, src, primary, blocks, timed,
+                  launches);
 }
 
-// One query batch `qb` on GPU x (its range of a multi-GPU batch) on stream st: the query's counters zeroed, the query
-// kernel of the ray type and, with hand-off, k_coop_query around it (traverse).  Closest hits use the work cursor and
-// hand-off line of launch 0, shadow queries those of launch CRT_MAX_LEVELS, as k_coop_query reads them.
+// One query batch `qb` on GPU x (its range of a multi-GPU batch) on stream st: the query's counters zeroed, then
+// traverse over the batch at level 0 (a zero Frame).  Closest hits use the work cursor and hand-off line of launch 0,
+// shadow queries those of launch CRT_MAX_LEVELS.
 static int enqueue_query(Gpu &x, const Flavour &fl, uint32_t ray_type, const QueryBatch &qb, cudaStream_t st,
                          uint32_t &launches) {
   QueueSet &q = x.query;
@@ -1666,29 +1655,12 @@ static int enqueue_query(Gpu &x, const Flavour &fl, uint32_t ray_type, const Que
   q.lv.tail_small = (uint32_t)x.tail_small;
   CUDA_TRY(cudaMemsetAsync(q.ctl.p, 0, q.ctl.n * sizeof(uint32_t), st));
   CUDA_TRY(cudaMemsetAsync(x.query_stats_dev.p, 0, CRT_STAT_SLOTS * sizeof(unsigned long long), st));
-  const bool shadow = ray_type == CRTB200_RAY_SHADOW, primary = ray_type == CRTB200_RAY_PRIMARY;
-  uint32_t *const work = q.work + CRT_CTL_STRIDE * (shadow ? (uint32_t)CRT_MAX_LEVELS : 0u);
   launches++;
-  return traverse(x, fl.handoff, true, q, st, shadow, 0, nullptr, launches, [&](cudaStream_t s, int coop_blocks, uint32_t early) {
-    if (coop_blocks) {
-      as_const(shadow, [&](auto sh) { as_const(primary, [&](auto prim) {
-        if constexpr (!(sh && prim)) k_coop_query<sh, prim><<<coop_blocks, 32 * CRT_COOP_WARPS, 0, s>>>(x.sc, q.lv, qb, early);
-      }); });
-    } else if (shadow) {
-      as_const_count(fl.count_work, [&](auto count) { as_const(fl.cull, [&](auto cull) { as_const(fl.wide_shadow, [&](auto wide) {
-        if constexpr (count != 1 || !(cull || wide))
-          k_query_shadow<count, CRT_REFILL_SHADOW, cull, wide>
-              <<<x.blocks_query_shadow, CRT_TRAV_BLOCK, wide ? dyn_smem(x, CRT_TRAV_BLOCK) : 0, s>>>(x.sc, q.lv, qb, work);
-      }); }); });
-    } else {
-      as_const(fl.count_work != 0, [&](auto count) { as_const(fl.cull, [&](auto cull) { as_const(fl.wide_closest, [&](auto wide) {
-        as_const(primary, [&](auto prim) {
-          if constexpr (!(count && wide))
-            k_query_closest<prim, count, CRT_REFILL_CLOSEST, cull, wide>
-                <<<x.blocks_query_closest, CRT_TRAV_BLOCK, dyn_smem(x, CRT_TRAV_BLOCK), s>>>(x.sc, q.lv, qb, work);
-        }); }); }); });
-    }
-  });
+  const Frame fr{};
+  if (ray_type == CRTB200_RAY_SHADOW)
+    return traverse(x, fl, true, q, st, fr, 0, QueryShadow{qb}, false, x.blocks_query_shadow, nullptr, launches);
+  return traverse(x, fl, true, q, st, fr, 0, QueryClosest{qb}, ray_type == CRTB200_RAY_PRIMARY, x.blocks_query_closest, nullptr,
+                  launches);
 }
 
 // The query scratch of GPU x, allocated on first use: work cursors | hand-off counters (ctl, the layout of a frame's
@@ -1698,9 +1670,9 @@ static int query_scratch(Gpu &x) {
   QueueSet &q = x.query;
   if (x.query_ready) return CRTB200_OK;
   int occ = 0;
-  CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_query_closest<true, false, CRT_REFILL_CLOSEST, true, false>, CRT_TRAV_BLOCK, 0));
+  CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_closest<QueryClosest, true, false, CRT_REFILL_CLOSEST, CRT_LOOP_MODE, true, false>, CRT_TRAV_BLOCK, 0));
   x.blocks_query_closest = std::max(1, occ) * x.sm_count;
-  CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_query_shadow<0, CRT_REFILL_SHADOW, true, false>, CRT_TRAV_BLOCK, 0));
+  CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_shadow<QueryShadow, 0, CRT_REFILL_SHADOW, CRT_LOOP_MODE, true, false>, CRT_TRAV_BLOCK, 0));
   x.blocks_query_shadow = std::max(1, occ) * x.sm_count;
   const uint64_t lanes = (uint64_t)std::max(x.blocks_query_closest, x.blocks_query_shadow) * CRT_TRAV_BLOCK;
   const uint64_t cap = std::min<uint64_t>(lanes, (uint64_t)x.tail_cap * x.blocks_coop * CRT_COOP_WARPS);
@@ -1779,9 +1751,11 @@ static Frame frame_tiles(const Gpu &g, uint32_t index, uint32_t count) {
 }
 
 // One sample pass of one chunk (sample fr.sample): the level loop, the shadow pass, k_accumulate, k_resolve and the
-// kernel that ends a sample of a GI frame or a progressive step
-static int sample_pass(Gpu &g, const FrameReq &r, const Flavour &fl, Frame &fr, QueueSet &q, uint32_t levels,
-                       crtb200_ctx *timed, uint32_t &launches) {
+// kernel that ends a sample of a GI frame or a progressive step.  Level 0 reads the request's source l0 (CameraRays or
+// ShadeRays); primary0: its rays take the primary ray's back-face rule.
+template <class L0>
+static int sample_pass(Gpu &g, const FrameReq &r, const Flavour &fl, Frame &fr, QueueSet &q, uint32_t levels, const L0 &l0,
+                       bool primary0, crtb200_ctx *timed, uint32_t &launches) {
   const cudaStream_t qs = q.stream;
   const int grid_simple = g.sm_count * 8;
   const bool adapt_step = r.acc && r.acc->ap;
@@ -1800,33 +1774,35 @@ static int sample_pass(Gpu &g, const FrameReq &r, const Flavour &fl, Frame &fr, 
   q.lv.tail_start = (uint32_t)g.tail_start;
   q.lv.tail_start_closest = (uint32_t)g.tail_start_closest;
   q.lv.tail_small = (uint32_t)g.tail_small;
+  // (levels above 0 read the queue, whatever the request's level 0: k_shade / k_resolve over CameraRays run them)
   for (uint32_t l = 0; l < levels; l++) {
-    const int rc = traverse_frame(g, fl, fr, q, false, l, timed, launches);
+    const int rc = l == 0 ? traverse_frame(g, fl, fr, q, 0, l0, primary0, timed, launches)
+                          : traverse_frame(g, fl, fr, q, l, QueueRays{}, false, timed, launches);
     if (rc) return rc;
     as_const(fl.gi, [&](auto gi) {
-      if (fl.rays && l == 0)
-        k_shade_rays<gi><<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, *fl.rays);
+      if (l == 0)
+        k_shade<gi><<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, 0u, l0);
       else
-        k_shade<gi><<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, l);
+        k_shade<gi><<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, l, CameraRays{});
     });
     launches += 2;
   }
-  const int rc = traverse_frame(g, fl, fr, q, true, 0, timed, launches);
+  const int rc = traverse_frame(g, fl, fr, q, 0, ShadowPairs{}, false, timed, launches);
   if (rc) return rc;
   k_accumulate<<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv);
   launches += 2;
   // (GI frames resolve the last level too: its diffuse hits combine D with G background children)
   for (uint32_t l = fl.gi ? levels : levels - 1; l-- > 0;) {
     as_const(fl.gi, [&](auto gi) {
-      if (fl.rays && l == 0)
-        k_resolve_rays<gi><<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, *fl.rays);
+      if (l == 0)
+        k_resolve<gi><<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, 0u, l0);
       else
-        k_resolve<gi><<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, l);
+        k_resolve<gi><<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, l, CameraRays{});
     });
     launches++;
   }
   // (a batch of caller rays is one pass with an arbitrary sample word: nothing to average)
-  const bool sample_acc = fl.gi && !fl.rays;
+  const bool sample_acc = fl.gi && std::is_same<L0, CameraRays>::value;
   if (adapt_step)
     k_adapt_step<<<grid_simple, 256, 0, qs>>>(g.sc, fr, q.lv, *r.acc->ap, g.acc_sum.p, g.acc_sumsq.p, g.acc_hit.p);
   else if (r.acc)
@@ -1877,8 +1853,7 @@ static int enqueue_frame(crtb200_ctx *c, Gpu &g, const FrameReq &r, cudaStream_t
   if (o->n_rects && !o->rects) return fail(CRTB200_ERR_ARG, "n_rects > 0 but rects is null");
   if (o->traversal > 1) return fail(CRTB200_ERR_ARG, "unknown traversal mode");
   if (o->count_work > 2) return fail(CRTB200_ERR_ARG, "unknown count_work mode");
-  Flavour fl = frame_flavour(g, o, r.sampling);
-  fl.rays = r.rays;
+  const Flavour fl = frame_flavour(g, o, r.sampling);
   const uint32_t shard_count = o->shard_count ? o->shard_count : 1;
   if (o->shard_index >= shard_count) return fail(CRTB200_ERR_ARG, "shard_index >= shard_count");
   int rc = r.rays ? CRTB200_OK : plan_mask(g, o);
@@ -1953,7 +1928,8 @@ static int enqueue_frame(crtb200_ctx *c, Gpu &g, const FrameReq &r, cudaStream_t
     }
     for (uint32_t k = 0; k < n_passes; k++) {
       fr.sample = s_begin + k;
-      rc = sample_pass(g, r, fl, fr, q, levels, timed, launches);
+      rc = r.rays ? sample_pass(g, r, fl, fr, q, levels, *r.rays, r.rays->stat == CRT_STAT_RAYS_PRIMARY, timed, launches)
+                  : sample_pass(g, r, fl, fr, q, levels, CameraRays{}, true, timed, launches);
       if (rc) return rc;
     }
     if (r.rays) {

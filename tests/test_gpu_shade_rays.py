@@ -209,7 +209,7 @@ def test_gi_samples_give_the_frame(gpu, loaded, crt, torch):
 @pytest.mark.parametrize("name", ["hw14_small", "hw11_room", "many_meshes"])
 def test_handoff_settings(name, which, handoff, loaded, crt, torch):
     """Forced, mid-flight, final-pass-only, capped and no hand-off: the oracle's colours; under "all" the level-0
-    walks went through k_coop_rays, under "off" nothing was handed off."""
+    walks went through k_coop over the caller's rays (ShadeRays), under "off" nothing was handed off."""
     ctx = handoff(which)
     sf, flat, _, _ = loaded[name]
     ctx.upload(flat, keepalive=sf)
