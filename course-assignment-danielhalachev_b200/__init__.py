@@ -254,6 +254,8 @@ def core() -> C.CDLL:
         lib.crtb200_upload_geometry.argtypes = [C.c_void_p, C.POINTER(Scene)]
         lib.crtb200_scene_trees.argtypes = [C.c_void_p, C.POINTER(Trees)]
         lib.crtb200_debug_scene_layout.argtypes = [C.c_void_p, C.c_int, C.POINTER(SceneLayout)]
+        lib.crtb200_update_vertices_device.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]
+        lib.crtb200_debug_scene_geometry.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
         lib.crtb200_set_sampling.argtypes = [C.c_void_p, C.POINTER(Sampling)]
         lib.crtb200_last_sampling_stats.argtypes = [C.c_void_p, C.POINTER(SamplingStats)]
         lib.crtb200_accum_begin.argtypes = [C.c_void_p, C.POINTER(Camera), C.POINTER(Options), C.POINTER(Sampling)]
@@ -382,6 +384,15 @@ class SceneFile:
             pass
 
 
+def scene_vertex_positions(scene_ptr) -> np.ndarray:
+    """A (n_vertices, 3) float32 copy of a flattened scene's vertex positions: the rest pose that Context.update_vertices
+    takes deformed."""
+    s = scene_ptr.contents
+    if s.n_vertices == 0:
+        return np.zeros((0, 3), np.float32)
+    return np.ctypeslib.as_array(s.vertex_position, shape=(s.n_vertices * 3,)).reshape(-1, 3).copy()
+
+
 def camera_pan(cam: Camera, degrees: float) -> Camera:
     _check_front(front().crtfe_camera_pan(C.byref(cam), degrees))
     return cam
@@ -452,6 +463,7 @@ class Context:
         else:
             _check_core(core().crtb200_create(int(device), C.byref(self._h)))
         self.width = self.height = 0
+        self.n_vertices = self.n_triangles = 0
         self._scene_keepalive = None
         self._session = None  # the Progressive whose session the context holds
 
@@ -468,6 +480,7 @@ class Context:
     def upload(self, scene_ptr, keepalive=None) -> None:
         _check_core(core().crtb200_upload_scene(self._h, scene_ptr))
         self.width, self.height = scene_ptr.contents.width, scene_ptr.contents.height
+        self.n_vertices, self.n_triangles = scene_ptr.contents.n_vertices, scene_ptr.contents.n_triangles
         self._scene_keepalive = keepalive
 
     def upload_geometry(self, scene_ptr, keepalive=None) -> None:
@@ -476,6 +489,7 @@ class Context:
         host-built trees leaves it."""
         _check_core(core().crtb200_upload_geometry(self._h, scene_ptr))
         self.width, self.height = scene_ptr.contents.width, scene_ptr.contents.height
+        self.n_vertices, self.n_triangles = scene_ptr.contents.n_vertices, scene_ptr.contents.n_triangles
         self._scene_keepalive = keepalive
 
     def scene_trees(self) -> dict:
@@ -506,6 +520,37 @@ class Context:
         _check_core(core().crtb200_debug_scene_layout(self._h, device_index, C.byref(l)))
         out.update(top_begin=l.top_begin, top_end=l.top_end, nested_ok=bool(l.nested_ok))
         return out
+
+    def update_vertices(self, positions) -> None:
+        """Moves the uploaded scene's vertices (crtb200_update_vertices_device): positions is a contiguous float32 CUDA
+        tensor of shape (n_vertices, 3) on the context's first device, read after the work already enqueued on
+        torch.cuda.current_stream().  Face and vertex normals are recomputed as Mesh::Mesh computes them and the KD trees
+        rebuilt on every GPU; afterwards the context is as upload_geometry of the scene with these positions leaves it,
+        except that the colour buffer keeps its pixels.  Returns once every GPU holds the new scene; a progressive
+        session ends."""
+        import torch
+        dev = self._first_device()
+        if not isinstance(positions, torch.Tensor):
+            raise CrtError("positions must be a torch tensor")
+        if positions.dtype != torch.float32:
+            raise CrtError(f"positions must be torch.float32, not {positions.dtype}")
+        if positions.device != dev:
+            raise CrtError(f"positions must be on {dev}, not {positions.device}")
+        if tuple(positions.shape) != (self.n_vertices, 3):
+            raise CrtError(f"positions must have shape {(self.n_vertices, 3)}, not {tuple(positions.shape)}")
+        if not positions.is_contiguous():
+            raise CrtError("positions must be contiguous")
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _check_core(core().crtb200_update_vertices_device(self._h, positions.data_ptr() or None, self.n_vertices, stream or None))
+
+    def debug_scene_geometry(self, device_index: int = 0):
+        """One GPU's triangle records and vertex normals (crtb200_debug_scene_geometry): (tri_geom (n_triangles, 3, 4)
+        float32 -- per corner the position and face-normal component k in the last column --, vertex_normal
+        (n_vertices, 3) float32)."""
+        geom = np.zeros((self.n_triangles, 3, 4), np.float32)
+        vn = np.zeros((self.n_vertices, 3), np.float32)
+        _check_core(core().crtb200_debug_scene_geometry(self._h, device_index, geom.ctypes.data, vn.ctypes.data))
+        return geom, vn
 
     def set_queue_budget(self, nbytes: int) -> None:
         _check_core(core().crtb200_set_queue_budget(self._h, nbytes))

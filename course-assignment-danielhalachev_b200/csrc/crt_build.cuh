@@ -506,4 +506,53 @@ __global__ void __launch_bounds__(256) k_build_margins(uint32_t n_meshes, const 
   meshes[m].cull_margin = mu_f;
 }
 
+// ---- vertex update: crtb200_update_vertices_device (DESIGN.md 3.14) --------------------------------------------------
+// Mesh::Mesh (Scene.cpp:5-30; csrc/frontend/crt_scene.cpp): per triangle n = cross(p1 - p0, p2 - p0), normalised; per
+// vertex the sum, from +0.0, of the face normals of its corners in (triangle, corner) order, normalised.
+
+// Per triangle: its three records of the build's triangle geometry (position, face normal component k in w), its face
+// normal, and its corners (key = vertex id, value = triangle) for the stable sort into the incidence list.
+__global__ void __launch_bounds__(256) k_update_tri_records(const float *__restrict__ pos, const uint4 *__restrict__ tri_shade,
+                                                            uint32_t n_tris, float4 *__restrict__ geom, float4 *__restrict__ face_n,
+                                                            uint32_t *__restrict__ corner_vtx, uint32_t *__restrict__ corner_tri) {
+  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n_tris) return;
+  const uint4 s = tri_shade[t];
+  const uint32_t iv[3] = {s.x, s.y, s.z};
+  V3 p[3];
+#pragma unroll
+  for (int k = 0; k < 3; k++) p[k] = mk(pos[3 * (size_t)iv[k]], pos[3 * (size_t)iv[k] + 1], pos[3 * (size_t)iv[k] + 2]);
+  const V3 n = vnorm(vcross(vsub(p[1], p[0]), vsub(p[2], p[0])));
+  const float nk[3] = {n.x, n.y, n.z};
+#pragma unroll
+  for (int k = 0; k < 3; k++) {
+    geom[3 * (size_t)t + k] = make_float4(p[k].x, p[k].y, p[k].z, nk[k]);
+    corner_vtx[3 * (size_t)t + k] = iv[k];
+    corner_tri[3 * (size_t)t + k] = t;
+  }
+  face_n[t] = make_float4(n.x, n.y, n.z, 0.f);
+}
+
+// Per vertex: its corners are the run of its id in the sorted keys (found by binary search); their face normals are
+// added in order to +0.0 (not started from the first term: +0 + -0 = +0 is what the reference computes), then
+// normalised.  A vertex no triangle references keeps (0, 0, 0).
+__global__ void __launch_bounds__(256) k_update_vertex_normals(const uint32_t *__restrict__ sorted_vtx, const uint32_t *__restrict__ sorted_tri,
+                                                               uint64_t n_corners, uint32_t n_vertices, const float4 *__restrict__ face_n,
+                                                               float4 *__restrict__ vtx_normal) {
+  const uint32_t v = blockIdx.x * blockDim.x + threadIdx.x;
+  if (v >= n_vertices) return;
+  uint64_t lo = 0, hi = n_corners;  // first corner with key >= v
+  while (lo < hi) {
+    const uint64_t mid = (lo + hi) >> 1;
+    if (sorted_vtx[mid] < v) lo = mid + 1; else hi = mid;
+  }
+  V3 sum = mk(0.0f, 0.0f, 0.0f);
+  for (uint64_t i = lo; i < n_corners && sorted_vtx[i] == v; i++) {
+    const float4 f = face_n[sorted_tri[i]];
+    sum = vadd(sum, mk(f.x, f.y, f.z));
+  }
+  sum = vnorm(sum);
+  vtx_normal[v] = make_float4(sum.x, sum.y, sum.z, 0.f);
+}
+
 }  // namespace crtd

@@ -20,6 +20,7 @@
 #include <string>
 #include <vector>
 
+#include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
 #include "../../include/crtb200.h"
@@ -305,6 +306,10 @@ struct crtb200_ctx {
   DevBuf<uint32_t> kd_refs;
   std::vector<crtb200_mesh> kd_meshes;
   crtb200_trees kd_counts{};
+  // the last upload's mesh records as given and its vertex count: crtb200_update_vertices_device rebuilds the trees
+  // over the same meshes
+  std::vector<crtb200_mesh> scene_meshes;
+  uint32_t n_vertices = 0;
 
   // frame, on the first GPU
   DevBuf<float> frame;   // persistent colour buffer (RayTracer::colorBuffer, RayTracer.h:69)
@@ -769,7 +774,12 @@ int crtb200_upload_scene(crtb200_ctx *c, const crtb200_scene *s) {
   c->kd_nodes.release();
   c->kd_refs.release();
   // scene replicated on every GPU (SURVEY 8(e)); the host relayout runs once per GPU, in parallel
-  return on_all_devices(c, [&](size_t, Gpu &g) { return upload_one(c, g, s); });
+  const int rc = on_all_devices(c, [&](size_t, Gpu &g) { return upload_one(c, g, s); });
+  if (rc == CRTB200_OK) {
+    c->scene_meshes.assign(s->meshes, s->meshes + s->n_meshes);
+    c->n_vertices = s->n_vertices;
+  }
+  return rc;
 }
 
 int crtb200_upload_geometry(crtb200_ctx *c, const crtb200_scene *s) {
@@ -788,6 +798,9 @@ int crtb200_upload_geometry(crtb200_ctx *c, const crtb200_scene *s) {
     c->trees_built = false;
     c->kd_nodes.release();
     c->kd_refs.release();
+  } else {
+    c->scene_meshes.assign(s->meshes, s->meshes + s->n_meshes);
+    c->n_vertices = s->n_vertices;
   }
   return rc;
 }
@@ -904,10 +917,30 @@ static int place_arena(Gpu &g, size_t n_nodes, size_t n_refs, size_t n_geom) {
   return CRTB200_OK;
 }
 
-// Uploads the records to GPU g and sets its device scene, and on the context's first GPU the frame buffers; the trees
-// (arena nodes and references, top_refs, meshes, nested_ok) are in place.
-static int commit_scene(crtb200_ctx *c, Gpu &g, const crtb200_scene *s, const SceneRecords &r, uint32_t n_nodes, uint32_t n_refs,
-                        uint32_t n_top_refs, uint32_t top_begin, uint32_t top_end) {
+// The trees' part of GPU g's device scene, once the arena (nodes, references, triangle records), top_refs and meshes
+// hold them: pointers, counts, the top-level tree's node range and the nesting flag.
+static void commit_trees(Gpu &g, uint32_t n_meshes, uint32_t n_nodes, uint32_t n_refs, uint32_t n_top_refs, uint32_t top_begin,
+                         uint32_t top_end, bool nested_ok) {
+  g.n_nodes = n_nodes;
+  g.n_leaf_refs = n_refs;
+  g.n_top_refs = n_top_refs;
+  g.nested_ok = nested_ok;
+  DScene &d = g.sc;
+  d.nodes = g.nodes_p;
+  d.leaf_refs = g.leaf_refs_p;
+  d.top_refs = g.top_refs.p;
+  d.tri_geom = g.tri_geom_p;
+  d.meshes = g.meshes.p;
+  d.n_meshes = n_meshes;
+  d.top_begin = top_begin;
+  d.top_end = top_end;
+  d.dedup_meshes = n_meshes <= 64 ? 1u : (n_meshes <= 512 ? 2u : 0u);
+  d.dedup_words = d.dedup_meshes == 2u ? (n_meshes + 31u) / 32u : 0u;
+}
+
+// Uploads the records to GPU g and completes its device scene, and on the context's first GPU the frame buffers; the
+// trees are committed (commit_trees).
+static int commit_records(crtb200_ctx *c, Gpu &g, const crtb200_scene *s, const SceneRecords &r) {
   g.has_reflective = g.has_refractive = false;
   for (uint32_t m = 0; m < s->n_meshes; m++) {
     const uint32_t type = s->materials[s->meshes[m].material].type;
@@ -922,32 +955,19 @@ static int commit_scene(crtb200_ctx *c, Gpu &g, const crtb200_scene *s, const Sc
   CUDA_TRY(g.texels.upload(r.texels));
   CUDA_TRY(g.lights.upload(r.lights));
   g.n_triangles = s->n_triangles;
-  g.n_nodes = n_nodes;
-  g.n_leaf_refs = n_refs;
-  g.n_top_refs = n_top_refs;
 
   DScene &d = g.sc;
-  d.nodes = g.nodes_p;
-  d.leaf_refs = g.leaf_refs_p;
-  d.top_refs = g.top_refs.p;
-  d.tri_geom = g.tri_geom_p;
   d.tri_shade = g.tri_shade.p;
   d.vtx_normal = g.vtx_normal.p;
   d.vtx_uv = r.uv.empty() ? nullptr : g.vtx_uv.p;
-  d.meshes = g.meshes.p;
   d.materials = g.materials.p;
   d.textures = g.textures.p;
   d.texels = g.texels.p;
   d.lights = g.lights.p;
   d.n_lights = s->n_lights;
-  d.n_meshes = s->n_meshes;
-  d.top_begin = top_begin;
-  d.top_end = top_end;
   d.width = s->width;
   d.height = s->height;
   for (int k = 0; k < 3; k++) d.bg[k] = s->background[k];
-  d.dedup_meshes = s->n_meshes <= 64 ? 1u : (s->n_meshes <= 512 ? 2u : 0u);
-  d.dedup_words = d.dedup_meshes == 2u ? (s->n_meshes + 31u) / 32u : 0u;
 
   const size_t px = (size_t)s->width * s->height;
   if (&g == c->gpus[0].get()) {
@@ -1021,10 +1041,10 @@ static int upload_one(crtb200_ctx *c, Gpu &g, const crtb200_scene *s) {
   if (!nodes.empty()) CUDA_TRY(cudaMemcpy(g.nodes_p, nodes.data(), nodes.size() * sizeof(float4), cudaMemcpyHostToDevice));
   if (!refs.empty()) CUDA_TRY(cudaMemcpy(g.leaf_refs_p, refs.data(), refs.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
   if (!r.geom.empty()) CUDA_TRY(cudaMemcpy(g.tri_geom_p, r.geom.data(), r.geom.size() * sizeof(float4), cudaMemcpyHostToDevice));
-  g.nested_ok = nested_ok;
   CUDA_TRY(g.top_refs.upload(top_refs));
   CUDA_TRY(g.meshes.upload(meshes));
-  return commit_scene(c, g, s, r, (uint32_t)(nodes.size() / 2), (uint32_t)refs.size(), (uint32_t)top_refs.size(), top_begin, top_end);
+  commit_trees(g, s->n_meshes, (uint32_t)(nodes.size() / 2), (uint32_t)refs.size(), (uint32_t)top_refs.size(), top_begin, top_end, nested_ok);
+  return commit_records(c, g, s, r);
 }
 
 // ---- device KD build: crtb200_upload_geometry (csrc/crt_build.cuh, DESIGN.md 3.11) -------------------------------
@@ -1081,37 +1101,38 @@ struct BuildAdd4 {
 
 static unsigned build_blocks(uint64_t n) { return (unsigned)std::max<uint64_t>(1, (n + 255) / 256); }
 
-// Builds the trees of `s` on GPU g of context c and uploads the scene; keep: also keep the reference-numbered trees for
-// crtb200_scene_trees.
-static int upload_geometry_one(crtb200_ctx *c, Gpu &g, const crtb200_scene *s, bool keep) {
-  SceneRecords r;
-  int rc = pack_records(g, s, false, r);
-  if (rc) return rc;
-  const uint32_t M = s->n_meshes, T = M + 1;
+static int build_nomem(const Gpu &g, const BuildScratch &sc) {
+  return fail(CRTB200_ERR_MEMORY, "device KD build: scratch does not fit on device " + std::to_string(g.device) + " (" +
+                                      std::to_string(sc.live) + " bytes allocated)");
+}
+
+// Builds the trees of M meshes (their first_triangle, n_triangles and material are read) over the n_tris triangle
+// records `geom` (3 per triangle, in sc on g's device, written on g's stream) on GPU g of context c, places the arena
+// (geom copied into it), top_refs and meshes with their culling margins, and commits them (commit_trees); keep: also
+// keep the reference-numbered trees for crtb200_scene_trees.  Shared by crtb200_upload_geometry and
+// crtb200_update_vertices_device.
+static int build_trees(crtb200_ctx *c, Gpu &g, const crtb200_mesh *in_meshes, uint32_t M, uint32_t n_tris, float4 *geom,
+                       BuildScratch &sc, bool keep) {
+  const uint32_t T = M + 1;
+  const size_t n_geom = 3 * (size_t)n_tris;
   std::vector<uint32_t> item_base(M + 1), mesh_tri(std::max(M, 1u), 0);
   uint64_t items = 0;
   for (uint32_t m = 0; m < M; m++) {
     item_base[m] = (uint32_t)std::min<uint64_t>(items, 0xFFFFFFFFu);
-    mesh_tri[m] = s->meshes[m].first_triangle;
-    items += s->meshes[m].n_triangles;
+    mesh_tri[m] = in_meshes[m].first_triangle;
+    items += in_meshes[m].n_triangles;
   }
   if (items + M >= 0x7FFFFFFFull) return fail(CRTB200_ERR_SCENE, "scene too large for 31-bit indices");
   item_base[M] = (uint32_t)items;
   const uint32_t NI = (uint32_t)items, NE = NI + M;
   cudaStream_t st = g.stream;
 
-  BuildScratch sc;
   bool ok = true;
   auto al = [&](auto *&p, size_t n) { ok = ok && sc.alloc(p, n); };
-  auto nomem = [&]() {
-    return fail(CRTB200_ERR_MEMORY, "device KD build: scratch does not fit on device " + std::to_string(g.device) + " (" +
-                                        std::to_string(sc.live) + " bytes allocated)");
-  };
-  float4 *geom;
+  auto nomem = [&]() { return build_nomem(g, sc); };
   uint32_t *d_item_base, *d_mesh_tri, *nested, *lelem, *lnode;
   BBox *ebox;
   unsigned long long *mslots, *slots;
-  al(geom, r.geom.size());
   al(d_item_base, M + 1);
   al(d_mesh_tri, mesh_tri.size());
   al(ebox, NE);
@@ -1143,7 +1164,6 @@ static int upload_geometry_one(crtb200_ctx *c, Gpu &g, const crtb200_scene *s, b
   CUDA_TRY(ev0.create(cudaEventDefault));
   CUDA_TRY(ev1.create(cudaEventDefault));
 
-  if (!r.geom.empty()) CUDA_TRY(cudaMemcpyAsync(geom, r.geom.data(), r.geom.size() * sizeof(float4), cudaMemcpyHostToDevice, st));
   CUDA_TRY(cudaMemcpyAsync(d_item_base, item_base.data(), item_base.size() * 4, cudaMemcpyHostToDevice, st));
   CUDA_TRY(cudaMemcpyAsync(d_mesh_tri, mesh_tri.data(), mesh_tri.size() * 4, cudaMemcpyHostToDevice, st));
   CUDA_TRY(cudaMemsetAsync(mslots, 0xFF, 6 * (size_t)T * sizeof(unsigned long long), st));
@@ -1261,16 +1281,16 @@ static int upload_geometry_one(crtb200_ctx *c, Gpu &g, const crtb200_scene *s, b
 
   // the scene's device arrays: arena, top-level references, meshes (the margins follow), kept trees
   CUDA_TRY(cudaStreamSynchronize(st));
-  rc = place_arena(g, n_nodes, n_refs, r.geom.size());
+  const int rc = place_arena(g, n_nodes, n_refs, n_geom);
   if (rc) return rc;
-  if (!r.geom.empty()) CUDA_TRY(cudaMemcpyAsync(g.tri_geom_p, geom, r.geom.size() * sizeof(float4), cudaMemcpyDeviceToDevice, st));
+  if (n_geom) CUDA_TRY(cudaMemcpyAsync(g.tri_geom_p, geom, n_geom * sizeof(float4), cudaMemcpyDeviceToDevice, st));
   CUDA_TRY(g.top_refs.ensure(std::max<uint32_t>(n_top_refs, 1)));
   std::vector<DMesh> meshes(M);
   for (uint32_t m = 0; m < M; m++) {
     meshes[m].node_begin = node_base[m];
     meshes[m].node_end = node_base[m] + root_size[m];
-    meshes[m].material = s->meshes[m].material;
-    meshes[m].first_triangle = s->meshes[m].first_triangle;
+    meshes[m].material = in_meshes[m].material;
+    meshes[m].first_triangle = in_meshes[m].first_triangle;
     meshes[m].cull_margin = std::numeric_limits<float>::infinity();
   }
   CUDA_TRY(g.meshes.upload(meshes));
@@ -1297,10 +1317,9 @@ static int upload_geometry_one(crtb200_ctx *c, Gpu &g, const crtb200_scene *s, b
   CUDA_TRY(cudaStreamSynchronize(st));
   float build_ms = 0.f;
   cudaEventElapsedTime(&build_ms, ev0, ev1);
-  g.nested_ok = nested_h != 0;  // every tree is at most 26 levels deep: k_coop's limit of 40 always holds
 
   if (keep) {
-    c->kd_meshes.assign(s->meshes, s->meshes + M);
+    c->kd_meshes.assign(in_meshes, in_meshes + M);
     for (uint32_t m = 0; m < M; m++) {
       c->kd_meshes[m].first_node = node_base[m];
       c->kd_meshes[m].n_nodes = root_size[m];
@@ -1317,10 +1336,108 @@ static int upload_geometry_one(crtb200_ctx *c, Gpu &g, const crtb200_scene *s, b
     k.peak_scratch_bytes = sc.peak;
     k.build_ms = build_ms;
   }
-  rc = commit_scene(c, g, s, r, (uint32_t)n_nodes, (uint32_t)n_refs, n_top_refs, top_begin, (uint32_t)n_nodes);
+  // every tree is at most 26 levels deep: k_coop's limit of 40 always holds
+  commit_trees(g, M, (uint32_t)n_nodes, (uint32_t)n_refs, n_top_refs, top_begin, (uint32_t)n_nodes, nested_h != 0);
+  return CRTB200_OK;
+}
+
+// Builds the trees of `s` on GPU g of context c and uploads the scene; keep: also keep the reference-numbered trees for
+// crtb200_scene_trees.
+static int upload_geometry_one(crtb200_ctx *c, Gpu &g, const crtb200_scene *s, bool keep) {
+  SceneRecords r;
+  int rc = pack_records(g, s, false, r);
+  if (rc) return rc;
+  BuildScratch sc;
+  float4 *geom;
+  if (!sc.alloc(geom, r.geom.size())) return build_nomem(g, sc);
+  if (!r.geom.empty()) CUDA_TRY(cudaMemcpyAsync(geom, r.geom.data(), r.geom.size() * sizeof(float4), cudaMemcpyHostToDevice, g.stream));
+  rc = build_trees(c, g, s->meshes, s->n_meshes, s->n_triangles, geom, sc, keep);
+  if (rc) return rc;
+  rc = commit_records(c, g, s, r);
   if (rc == CRTB200_OK && keep) c->trees_built = true;
   return rc;
 }
+
+// GPU g's part of crtb200_update_vertices_device, once the caller's stream reached `fork`: the positions (GPUs after
+// the first copy them from the first GPU), the triangle records and face normals, the incidence list (corners sorted
+// stably by vertex id) and the vertex normals, then the build.  The old scene is gone from the first write on.
+static int update_one(crtb200_ctx *c, Gpu &g, const float *d_positions, uint32_t n_vertices, cudaEvent_t fork, bool keep) {
+  CUDA_TRY(cudaSetDevice(g.device));
+  g.have_scene = false;
+  cudaStream_t st = g.stream;
+  CUDA_TRY(cudaStreamWaitEvent(st, fork, 0));
+  const uint32_t T = g.n_triangles, V = n_vertices;
+  const uint64_t NC = 3 * (uint64_t)T;
+  BuildScratch sc;
+  const float *pos = d_positions;
+  float *pos_copy = nullptr;
+  if (&g != c->gpus[0].get() && V) {
+    if (!sc.alloc(pos_copy, 3 * (size_t)V)) return build_nomem(g, sc);
+    CUDA_TRY(cudaMemcpyPeerAsync(pos_copy, g.device, d_positions, c->gpus[0]->device, 3 * (size_t)V * sizeof(float), st));
+    pos = pos_copy;
+  }
+  float4 *geom, *face_n;
+  uint32_t *corner_vtx, *corner_tri, *sorted_vtx, *sorted_tri;
+  if (!sc.alloc(geom, NC) || !sc.alloc(face_n, T) || !sc.alloc(corner_vtx, NC) || !sc.alloc(corner_tri, NC) ||
+      !sc.alloc(sorted_vtx, NC) || !sc.alloc(sorted_tri, NC))
+    return build_nomem(g, sc);
+  int end_bit = 1;  // the sort's key bits: enough for the largest vertex id
+  while (end_bit < 32 && ((V - 1u) >> end_bit)) end_bit++;
+  size_t cub_bytes = 0;
+  CUDA_TRY(cub::DeviceRadixSort::SortPairs(nullptr, cub_bytes, corner_vtx, sorted_vtx, corner_tri, sorted_tri, NC, 0, end_bit, st));
+  uint8_t *cub_tmp;
+  if (!sc.alloc(cub_tmp, cub_bytes)) return build_nomem(g, sc);
+  if (T) {
+    k_update_tri_records<<<build_blocks(T), 256, 0, st>>>(pos, g.tri_shade.p, T, geom, face_n, corner_vtx, corner_tri);
+    CUDA_TRY(cub::DeviceRadixSort::SortPairs(cub_tmp, cub_bytes, corner_vtx, sorted_vtx, corner_tri, sorted_tri, NC, 0, end_bit, st));
+  }
+  if (V) k_update_vertex_normals<<<build_blocks(V), 256, 0, st>>>(sorted_vtx, sorted_tri, NC, V, face_n, g.vtx_normal.p);
+  CUDA_TRY(cudaGetLastError());
+  for (void *p : {(void *)cub_tmp, (void *)sorted_tri, (void *)sorted_vtx, (void *)corner_tri, (void *)corner_vtx, (void *)face_n, (void *)pos_copy})
+    if (p) sc.free(p);
+  const int rc = build_trees(c, g, c->scene_meshes.data(), (uint32_t)c->scene_meshes.size(), T, geom, sc, keep);
+  if (rc) return rc;
+  g.have_scene = true;
+  if (keep) c->trees_built = true;
+  return CRTB200_OK;
+}
+
+static int check_device_ptr(const Gpu &g, const void *p, size_t align, const char *what);
+
+extern "C" {
+
+int crtb200_update_vertices_device(crtb200_ctx *c, const float *d_positions, uint32_t n_vertices, void *stream) {
+  if (!c) return fail(CRTB200_ERR_ARG, "null argument");
+  ErrScope scope(c);
+  for (auto &g : c->gpus)
+    if (!g->have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
+  if (n_vertices != c->n_vertices)
+    return fail(CRTB200_ERR_ARG, "n_vertices is " + std::to_string(n_vertices) + ", the uploaded scene has " + std::to_string(c->n_vertices));
+  Gpu &g0 = *c->gpus[0];
+  CUDA_TRY(cudaSetDevice(g0.device));
+  if (n_vertices) {
+    const int rc = check_device_ptr(g0, d_positions, 4, "positions");
+    if (rc) return rc;
+  }
+  if (c->acc_active) accum_release(c);
+  c->trees_built = false;
+  c->kd_nodes.release();
+  c->kd_refs.release();
+  // every GPU starts once the work enqueued on the caller's stream so far (renders, queries, the positions' writes) is done
+  Event fork;
+  CUDA_TRY(fork.create(cudaEventDisableTiming));
+  CUDA_TRY(cudaEventRecord(fork, (cudaStream_t)stream));
+  const int rc = on_all_devices(c, [&](size_t i, Gpu &g) { return update_one(c, g, d_positions, n_vertices, fork, i == 0); });
+  if (rc) {
+    c->trees_built = false;
+    c->kd_nodes.release();
+    c->kd_refs.release();
+  }
+  cudaSetDevice(g0.device);
+  return rc;
+}
+
+}  // extern "C"
 
 // ---- frame planning ------------------------------------------------------------------------------------------
 // worst-case children of one ray-tree node: refractive hits spawn two (RayTracer.cpp:398-412), reflective ones one, and
@@ -2725,6 +2842,25 @@ int crtb200_debug_scene_layout(crtb200_ctx *c, int device_index, crtb200_scene_l
   get(l->leaf_refs, x.leaf_refs_p, (size_t)x.n_leaf_refs * 4);
   get(l->top_refs, x.top_refs.p, (size_t)x.n_top_refs * 4);
   get(l->meshes, x.meshes.p, (size_t)x.sc.n_meshes * sizeof(DMesh));
+  if (e == cudaSuccess) e = cudaStreamSynchronize(x.stream);
+  cudaSetDevice(c->gpus[0]->device);
+  CUDA_TRY(e);
+  return CRTB200_OK;
+}
+
+int crtb200_debug_scene_geometry(crtb200_ctx *c, int device_index, float *tri_geom_out, float *vertex_normal_out) {
+  ErrScope scope(c);
+  if (!c) return fail(CRTB200_ERR_ARG, "null argument");
+  if (device_index < 0 || (size_t)device_index >= c->gpus.size()) return fail(CRTB200_ERR_ARG, "device_index out of range");
+  Gpu &x = *c->gpus[device_index];
+  if (!x.have_scene) return fail(CRTB200_ERR_STATE, "no scene uploaded");
+  CUDA_TRY(cudaSetDevice(x.device));
+  cudaError_t e = cudaSuccess;
+  if (tri_geom_out && x.n_triangles)
+    e = cudaMemcpyAsync(tri_geom_out, x.tri_geom_p, (size_t)x.n_triangles * 3 * sizeof(float4), cudaMemcpyDeviceToHost, x.stream);
+  if (vertex_normal_out && c->n_vertices && e == cudaSuccess)  // float4 (n, 0) per vertex -> 3 floats
+    e = cudaMemcpy2DAsync(vertex_normal_out, 3 * sizeof(float), x.vtx_normal.p, sizeof(float4), 3 * sizeof(float), c->n_vertices,
+                          cudaMemcpyDeviceToHost, x.stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(x.stream);
   cudaSetDevice(c->gpus[0]->device);
   CUDA_TRY(e);

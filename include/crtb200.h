@@ -261,7 +261,7 @@ int crtb200_last_sampling_stats(crtb200_ctx *ctx, crtb200_sampling_stats *stats)
  * crtb200_accum_read returns bit for bit what crtb200_render returns with the same camera and options and
  * rays_per_pixel = n, and the steps' ray counts (and, with count_work = 1, test counts) add up to that frame's.
  * Ordinary renders and crtb200_set_sampling between steps do not affect the session; crtb200_upload_scene,
- * crtb200_upload_geometry and crtb200_destroy end it.  Every call but begin fails with CRTB200_ERR_STATE without a session. */
+ * crtb200_upload_geometry, crtb200_update_vertices_device and crtb200_destroy end it.  Every call but begin fails with CRTB200_ERR_STATE without a session. */
 
 /* replaces: the per-pixel sample loop's set-up, RayTracer.cpp:90-104 (no counterpart: see above).  Snapshots camera,
  * options (the rects array is copied) and sampling (rays_per_pixel is ignored) and starts at 0 samples; a session in
@@ -355,8 +355,8 @@ typedef struct crtb200_trees {
   uint32_t *top_leaf_refs;     /* n_top_leaf_refs mesh indices                                                      */
 } crtb200_trees;
 /* replaces: the AccelerationStructure a RayTracer holds (RayTracer.h:65), read back.  Fills the counts, then every
- * non-NULL array (sized from a call with NULL arrays).  CRTB200_ERR_STATE unless the context's scene came from
- * crtb200_upload_geometry. */
+ * non-NULL array (sized from a call with NULL arrays).  CRTB200_ERR_STATE unless the context's trees were built on the
+ * device: by crtb200_upload_geometry or crtb200_update_vertices_device. */
 int crtb200_scene_trees(crtb200_ctx *ctx, crtb200_trees *trees);
 
 /* The device scene state of one GPU of the context, as the traversal kernels read it (csrc/crt_device.cuh). */
@@ -374,6 +374,27 @@ typedef struct crtb200_scene_layout {
  * every non-NULL array -- so tests can compare crtb200_upload_geometry with crtb200_upload_scene bit for bit.
  * CRTB200_ERR_STATE without a scene. */
 int crtb200_debug_scene_layout(crtb200_ctx *ctx, int device_index, crtb200_scene_layout *layout);
+
+/* replaces: rebuilding a RayTracer for a scene whose vertices moved -- Mesh::Mesh's face and vertex normals
+ * (Scene.cpp:5-30) and TriangleKDTree / ObjectKDTree (AccelerationStructure.cpp:12-50) -- from DEVICE memory
+ * (DESIGN.md 3.14).  d_positions holds n_vertices * 3 float32 in device memory of the context's first GPU, 4-byte
+ * aligned; n_vertices must be the uploaded scene's vertex count (0 for a scene without vertices: d_positions may then
+ * be NULL).  Afterwards every GPU of the context holds exactly what crtb200_upload_geometry leaves for the uploaded
+ * scene with these positions, its triangle and vertex normals as Mesh::Mesh computes them from these positions (in
+ * binary32 without contraction), and everything else unchanged; crtb200_scene_trees then describes the new trees and
+ * this build, whichever upload the scene came from.  The positions are read after the work already enqueued on `stream`
+ * (a cudaStream_t, NULL = default), so renders, queries and shades enqueued there before finish first; work of this
+ * context on other streams is the caller's to order, as for uploads.  Synchronous: on return every GPU holds the new
+ * scene and d_positions may be overwritten.  Ends a progressive session.  Unlike an upload it keeps the colour buffer
+ * (pixels outside a later render's rects keep their values, as across camera moves), and it leaves
+ * crtb200_last_stats, the sampling stats and crtb200_last_query_stats alone.
+ * CRTB200_ERR_STATE without a scene.  CRTB200_ERR_ARG: null positions with n_vertices > 0, positions not device memory
+ * of the first GPU or misaligned, a wrong n_vertices.  CRTB200_ERR_MEMORY when the build's scratch does not fit.  A
+ * failure after the update began leaves the context without a scene, as a failed crtb200_upload_geometry does. */
+int crtb200_update_vertices_device(crtb200_ctx *ctx, const float *d_positions, uint32_t n_vertices, void *stream);
+/* Test hook: GPU device_index's triangle records (n_triangles * 12 float32: p0.xyz, n.x, p1.xyz, n.y, p2.xyz, n.z, the
+ * tri_geom layout) and vertex normals (n_vertices * 3), each optional.  CRTB200_ERR_STATE without a scene. */
+int crtb200_debug_scene_geometry(crtb200_ctx *ctx, int device_index, float *tri_geom_out, float *vertex_normal_out);
 
 /* replaces: RayTracer::render's scheduler switch + renderRectangle pixel loop (RayTracer.cpp:82-112,209-286).
  * rgb_out: H*W*3 float32 row-major, host memory, = the colorBuffer render() returns (RayTracer.cpp:297).  Pixels not
